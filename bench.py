@@ -13,6 +13,7 @@ is measured too and reported as the named extra `weak_scaling` (`--scaling weak`
 
   python bench.py --gpus N --steps K --warmup W            # B200 arm (libb200vo.so)
   python bench.py --impl reference --gpus N --steps K ...  # the reference's own cv2 CPU path
+  python bench.py --gpus 1 --steps K --dump-outputs DIR    # + the last timed step's results as DIR/<name>.npy
 
 Prints ONE JSON line on rank 0.  Everything that is not the headline (`single_sequence`, `detect`,
 `weak_scaling`, `parity`, `cpu_baseline`) is guarded: a failure there is recorded as {"error": ...}
@@ -58,6 +59,8 @@ def parse(argv=None):
     ap.add_argument("--no-weak", action="store_true", help="skip the extra 64-per-GPU (weak scaling) measurement at N > 1")
     ap.add_argument("--no-parity", action="store_true", help="skip the post-run oracle check of the last timed step")
     ap.add_argument("--no-lookahead", action="store_true", help="device-resident loop: pass each step's frames with the step instead of one step ahead")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the results of the last timed device-resident step to DIR/<name>.npy (rank 0's sequences)")
     return ap.parse_args(argv)
 
 
@@ -358,6 +361,9 @@ class Arm:
         self.barrier()
         dev_ms = e0.elapsed_time(e1)
         launches = ctx.launch_count() - launches0
+        # the results of the last timed step, read before the profiled pass below overwrites the output buffers
+        timed_last = ({k: (v[W + K - 1] if k == "pose" else v).cpu().numpy() for k, v in d_out.items()}
+                      if self.args.dump_outputs else None)
         # Per-launch stage times come from a SEPARATE pass of P more steps right behind the timed region: the timing events
         # b200vo_batch_profile puts between the launches stall this stream structure by ~0.1 ms in every other step (measured
         # with the kernels' own %globaltimer stamps, B200VO_TRACE_FILE: gaps of 8-10 us between launches without them, 100-145
@@ -375,7 +381,8 @@ class Arm:
         n_gathered = None if gathered is None else int(sum(int(g_.shape[0]) for g_ in gathered))
         last = {k: (v[W + K + P - 1] if k == "pose" else v).cpu().numpy() for k, v in d_out.items()}
         return {"dev_ms": dev_ms, "launches": int(launches), "stage_ms": stage_ms, "nprof": int(nprof[0]), "n_ok": n_ok,
-                "gathered_sequences": n_gathered, "last": last, "last_t": W + K + P - 1, "profiled_steps": P}
+                "gathered_sequences": n_gathered, "last": last, "last_t": W + K + P - 1, "profiled_steps": P,
+                "timed_last": timed_last, "timed_last_t": W + K - 1}
 
     # ---- (2) end to end through the C-ABI with HOST buffers (pinned; H2D + D2H inside the timed region) ----
     def host_buffers(self):
@@ -506,6 +513,37 @@ def parity_check(arm, res, n_check=2):
         ok_all = ok_all and bool(ok_s)
     out.update(ok=bool(ok_all), klt_max_abs_diff_px=max_d, pose_max_abs_diff=pose_d)
     return out
+
+
+DUMP_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(arm, res, out_dir):
+    """Writes what the last timed device-resident step returned to out_dir/<name>.npy (float32, pose float64), so that
+    two builds run with the same arguments can be compared output for output.  Point slots at or past a sequence's
+    point count hold no result and are written as 0; sequence_index is each row's global sequence index.  Above
+    DUMP_BYTES in all, a fixed seeded sample of the sequences is written."""
+    wl, last = arm.wl, res["timed_last"]
+    f = arm.fo(res["timed_last_t"])
+    lm_live = np.arange(wl.L)[None, :] < wl.n_lm[f][:, None]
+    cand_live = np.arange(wl.Cn)[None, :] < wl.n_cand[f][:, None]
+    out = {"lm_next": np.where(lm_live[..., None], last["lm_next"], 0).astype(np.float32),
+           "lm_status": np.where(lm_live, last["lm_status"], 0).astype(np.float32),
+           "cand_next": np.where(cand_live[..., None], last["cand_next"], 0).astype(np.float32),
+           "cand_status": np.where(cand_live, last["cand_status"], 0).astype(np.float32),
+           "pose": last["pose"].astype(np.float64),
+           "pnp_ok": last["pnp_ok"].astype(np.float32),
+           "inlier_mask": np.where(lm_live, last["inlier_mask"], 0).astype(np.float32),
+           "n_inliers": last["n_inliers"].astype(np.float32),
+           "sequence_index": np.arange(wl.first_index, wl.first_index + wl.batch, dtype=np.float64)}
+    per_sequence = sum(a.nbytes for a in out.values()) / wl.batch
+    keep = int((DUMP_BYTES - 128 * len(out)) // per_sequence)      # 128: header of one .npy file
+    if keep < wl.batch:
+        rows = np.sort(np.random.default_rng(0).choice(wl.batch, keep, replace=False))
+        out = {k: a[rows] for k, a in out.items()}
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in out.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
 
 
 def measure_detect(arm):
@@ -765,6 +803,8 @@ def main(argv=None):
         th.join(timeout=2)
     clocks = summarize_clocks(clk_samples)
 
+    if args.dump_outputs and rank == 0:
+        dump_outputs(arm, res, args.dump_outputs)
     roofline, levels = klt_roofline(args, opts, wl, res, ROOFLINE_NOTE)
     parity = None if args.no_parity or rank != 0 else guarded(parity_check, arm, res)
     solo = rank == 0 and world == 1 and not args.no_single
@@ -828,4 +868,5 @@ def main(argv=None):
 
 
 if __name__ == "__main__":
+    sys.dont_write_bytecode = True      # the benchmark leaves the tree as it found it (no __pycache__ of the modules it imports)
     main()

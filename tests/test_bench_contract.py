@@ -140,6 +140,59 @@ def test_host_loops_for_every_step_count(bench_mod, steps, warmup, prefetch):
     assert arm.sb.queued == 0 and arm.sb.steps == arm.K + arm.W + (1 if prefetch else 0)
 
 
+def _fake_step_results(wl, seed):
+    import numpy as np
+    rng = np.random.default_rng(seed)
+    b, L, Cn = wl.batch, wl.L, wl.Cn
+    return {"lm_next": rng.random((b, L, 2), np.float32), "lm_status": rng.integers(0, 2, (b, L), np.uint8),
+            "cand_next": rng.random((b, Cn, 2), np.float32), "cand_status": rng.integers(0, 2, (b, Cn), np.uint8),
+            "pose": rng.random((b, 6)), "pnp_ok": np.ones(b, np.uint8), "inlier_mask": rng.integers(0, 2, (b, L), np.uint8),
+            "n_inliers": rng.integers(0, L, b).astype(np.int32)}
+
+
+def test_dump_outputs_writes_the_last_timed_step(bench_mod, tmp_path):
+    import numpy as np
+    args = _small_args(bench_mod, 4, 3)
+    wl = bench_mod.make_workload(args, 2, 5)
+    arm = object.__new__(bench_mod.Arm)
+    arm.wl = wl
+    last = _fake_step_results(wl, 0)
+    t = 3 + 4 - 1
+    bench_mod.dump_outputs(arm, {"timed_last": last, "timed_last_t": t}, str(tmp_path))
+    f = arm.fo(t)
+    got = {p.stem: np.load(p) for p in tmp_path.glob("*.npy")}
+    assert sorted(got) == sorted(list(last) + ["sequence_index"])
+    assert all(a.dtype in (np.float32, np.float64) for a in got.values())
+    assert got["pose"].dtype == np.float64 and np.array_equal(got["pose"], last["pose"])
+    assert np.array_equal(got["sequence_index"], [5, 6]) and np.array_equal(got["n_inliers"], last["n_inliers"])
+    for s in range(wl.batch):
+        nl, nc = wl.n_lm[f, s], wl.n_cand[f, s]
+        assert np.array_equal(got["lm_next"][s, :nl], last["lm_next"][s, :nl]) and not got["lm_next"][s, nl:].any()
+        assert np.array_equal(got["lm_status"][s, :nl], last["lm_status"][s, :nl]) and not got["lm_status"][s, nl:].any()
+        assert np.array_equal(got["inlier_mask"][s, :nl], last["inlier_mask"][s, :nl]) and not got["inlier_mask"][s, nl:].any()
+        assert np.array_equal(got["cand_next"][s, :nc], last["cand_next"][s, :nc]) and not got["cand_next"][s, nc:].any()
+
+
+def test_dump_outputs_samples_sequences_above_the_size_limit(bench_mod, tmp_path, monkeypatch):
+    import numpy as np
+    args = _small_args(bench_mod, 4, 3)
+    wl = bench_mod.make_workload(args, 6, 0)
+    arm = object.__new__(bench_mod.Arm)
+    arm.wl = wl
+    last = _fake_step_results(wl, 1)
+    full = tmp_path / "full"
+    bench_mod.dump_outputs(arm, {"timed_last": last, "timed_last_t": 7}, str(full))
+    limit = sum(p.stat().st_size for p in full.glob("*.npy")) // 2
+    monkeypatch.setattr(bench_mod, "DUMP_BYTES", limit)
+    for run in ("a", "b"):
+        bench_mod.dump_outputs(arm, {"timed_last": last, "timed_last_t": 7}, str(tmp_path / run))
+        assert sum(p.stat().st_size for p in (tmp_path / run).glob("*.npy")) <= limit
+    rows = np.load(tmp_path / "a" / "sequence_index.npy").astype(int)
+    assert 0 < len(rows) < wl.batch and np.array_equal(rows, np.load(tmp_path / "b" / "sequence_index.npy"))
+    for p in full.glob("*.npy"):
+        assert np.array_equal(np.load(tmp_path / "a" / p.name), np.load(p)[rows]), p.name
+
+
 def test_frame_at_is_total_and_matches_frame_order():
     from monocular_visual_odometry_va4mr_b200 import workload
     for F in (1, 2, 3, 6):

@@ -1,9 +1,8 @@
-"""The UNMODIFIED reference class (/root/reference/VisualOdometryPipeLine.py) running on the CUDA path through
-`cv2_compat.install()` -- what "drop-in" means.  Needs both a B200 and the reference checkout: the GPU box has no
-/root/reference and the build container has no GPU, so the test skips unless someone provides both (set
-B200VO_REFERENCE_DIR to a checkout of the reference on a GPU machine).  The free-running GPU tests in
-test_free_running_gpu.py drive the same data flow through tests/mini_vo.py (a restatement that is itself pinned to
-the recorded reference run by test_oracle_free_running.py)."""
+"""The UNMODIFIED reference class (VisualOdometryPipeLine.py of ManuelWendl/Monocular_Visual_Odometry_VA4MR) running
+on the CUDA path through `cv2_compat.install()` -- what "drop-in" means.  The reference is not part of this
+repository, so the test needs a B200 and a checkout of the reference named by B200VO_REFERENCE_DIR, and skips
+without one.  The free-running GPU tests in test_free_running_gpu.py drive the same data flow through
+tests/mini_vo.py (a restatement that is itself pinned to the recorded reference run by test_oracle_free_running.py)."""
 import os
 import sys
 
@@ -13,10 +12,11 @@ import pytest
 from monocular_visual_odometry_va4mr_b200 import cv2_compat, synth
 
 pytestmark = pytest.mark.gpu
-REF = os.environ.get("B200VO_REFERENCE_DIR", "/root/reference")
+REF = os.environ.get("B200VO_REFERENCE_DIR", "")
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(REF, "VisualOdometryPipeLine.py")), reason="the reference checkout is not on this machine")
+@pytest.mark.skipif(not REF or not os.path.exists(os.path.join(REF, "VisualOdometryPipeLine.py")),
+                    reason="B200VO_REFERENCE_DIR does not name a checkout of the reference project")
 def test_unmodified_reference_class_runs_on_the_cuda_path():
     cv2 = pytest.importorskip("cv2")
     sys.path.insert(0, REF)
