@@ -68,10 +68,10 @@ struct b200vo_batch {
     bool prof_init = false;
 };
 
-static void prof_mark(b200vo_batch* B, int stage)
+static void prof_mark(b200vo_batch* B, int stage, cudaStream_t stream)
 {
     if (!B->profile || B->prof_n >= B200VO_PROF_RING) return;
-    cudaEventRecord(B->prof_ev[B->prof_n][stage], B->ctx->stream);
+    cudaEventRecord(B->prof_ev[B->prof_n][stage], stream);
 }
 
 // status==1 landmarks, in order, into the compact PnP input arrays (what `matched_pts[tracked]`
@@ -284,7 +284,7 @@ static int batch_upload_frames(b200vo_batch* B, const uint8_t* frames, int slab_
     }
     VO_CUDA(ctx, cudaMemcpyAsync(B->raw.p, src, total, cudaMemcpyHostToDevice, ctx->stream));
     VO_TRY(vo_build_pyramids(ctx, (const uint8_t*)B->raw.p, fb, B->cfg.rows, B->cfg.cols, B->geom,
-                             (uint8_t*)B->slabs[slab_set].p, B->geom.slab_bytes, B->batch));
+                             (uint8_t*)B->slabs[slab_set].p, B->geom.slab_bytes, B->batch, ctx->stream));
     return 0;
 }
 
@@ -356,12 +356,8 @@ static int batch_issue_prefetch(b200vo_batch* B, cudaEvent_t after = nullptr, bo
             VO_CUDA(ctx, cudaMemcpyAsync(B->raw_pre.p, B->q_src[slot], total, cudaMemcpyHostToDevice, B->pre_stream));
             raw = (const uint8_t*)B->raw_pre.p;
         }
-        cudaStream_t main_stream = ctx->stream;
-        ctx->stream = B->pre_stream;
-        const int rc = vo_build_pyramids(ctx, raw, fb, B->cfg.rows, B->cfg.cols, B->geom,
-                                         (uint8_t*)B->slabs[B->q_set[slot]].p, B->geom.slab_bytes, B->batch);
-        ctx->stream = main_stream;
-        if (rc) return rc;
+        VO_TRY(vo_build_pyramids(ctx, raw, fb, B->cfg.rows, B->cfg.cols, B->geom,
+                                 (uint8_t*)B->slabs[B->q_set[slot]].p, B->geom.slab_bytes, B->batch, B->pre_stream));
         VO_CUDA(ctx, cudaEventRecord(B->q_ev[slot], B->pre_stream));
         B->q_src[slot] = nullptr;
     }
@@ -383,11 +379,11 @@ extern "C" int b200vo_batch_prime(b200vo_batch* B, const uint8_t* frames)
 }
 
 // device-resident core: everything after the new frames are in `frames_dev`
-// pyramids of the new frames + KLT for sequences [b0, b0 + nb)
+// pyramids of the new frames + KLT for sequences [b0, b0 + nb), enqueued on `stream`
 // (frames_dev == nullptr: the pyramids of set B->nxt were built ahead by b200vo_batch_submit_frames)
 // which: 0 = pyramids + both point sets in one launch, 1 = landmark set only, 2 = candidate set only, 3 = pyramids only,
 // 4 = pyramids + landmark set
-static int batch_track(b200vo_batch* B, int b0, int nb, const uint8_t* frames_dev, const float* lm_pts, const int* n_lm,
+static int batch_track(b200vo_batch* B, cudaStream_t stream, int b0, int nb, const uint8_t* frames_dev, const float* lm_pts, const int* n_lm,
                        const float* cand_pts, const int* n_cand, float* lm_next, uint8_t* lm_status, float* cand_next,
                        uint8_t* cand_status, int which = 0)
 {
@@ -398,11 +394,11 @@ static int batch_track(b200vo_batch* B, int b0, int nb, const uint8_t* frames_de
     const int L = c.max_landmarks, Cn = c.max_candidates;
     if (which == 0 || which == 3 || which == 4) {
         const bool whole = b0 == 0 && nb == B->batch;   // chunked uploads build the pyramids piecewise: no single interval to time
-        if (whole) prof_mark(B, 0);
+        if (whole) prof_mark(B, 0, stream);
         if (frames_dev)
             VO_TRY(vo_build_pyramids(ctx, frames_dev + (size_t)b0 * fb, fb, c.rows, c.cols, B->geom,
-                                     (uint8_t*)B->slabs[nxt].p + (size_t)b0 * sb, sb, nb));
-        if (whole) { prof_mark(B, 1); B->prof_row_open = B->profile && B->prof_n < B200VO_PROF_RING; }
+                                     (uint8_t*)B->slabs[nxt].p + (size_t)b0 * sb, sb, nb, stream));
+        if (whole) { prof_mark(B, 1, stream); B->prof_row_open = B->profile && B->prof_n < B200VO_PROF_RING; }
     }
     KltPointSet sets[2] = {{L, n_lm + b0, lm_pts + (size_t)b0 * L * 2, lm_next + (size_t)b0 * L * 2, lm_status + (size_t)b0 * L, nullptr},
                            {Cn, n_cand + b0, cand_pts + (size_t)b0 * Cn * 2, cand_next + (size_t)b0 * Cn * 2,
@@ -411,17 +407,17 @@ static int batch_track(b200vo_batch* B, int b0, int nb, const uint8_t* frames_de
     const KltPointSet* first = which == 2 ? sets + 1 : sets;
     const int n_sets = which == 0 ? (Cn > 0 ? 2 : 1) : 1;   // which 1, 4: landmark set; 2: candidate set
     VO_TRY(vo_klt_launch2(ctx, B->geom, (const uint8_t*)B->slabs[B->cur].p + (size_t)b0 * sb, sb,
-                          (const uint8_t*)B->slabs[nxt].p + (size_t)b0 * sb, sb, nb, first, n_sets, 0, B->kp));
+                          (const uint8_t*)B->slabs[nxt].p + (size_t)b0 * sb, sb, nb, first, n_sets, 0, B->kp, stream));
     return 0;
 }
 
-// status==1 compaction, P3P-RANSAC + EPnP, inlier mask -- whole batch
-static int batch_pose(b200vo_batch* B, const float* lm_obj, const int* n_lm, const float* lm_next, const uint8_t* lm_status,
+// status==1 compaction, P3P-RANSAC + EPnP, inlier mask -- whole batch, enqueued on `stream`
+static int batch_pose(b200vo_batch* B, cudaStream_t stream, const float* lm_obj, const int* n_lm, const float* lm_next, const uint8_t* lm_status,
                       double* pose, uint8_t* pnp_ok, uint8_t* inlier_mask, int* n_inliers)
 {
     b200vo_ctx* ctx = B->ctx;
     const b200vo_batch_cfg& c = B->cfg;
-    if (B->prof_row_open) prof_mark(B, 2);
+    if (B->prof_row_open) prof_mark(B, 2, stream);
     PnpArgs a{};
     a.batch = B->batch; a.cap = c.max_landmarks; a.iters = c.pnp_iters;
     a.obj = B->c_obj; a.img = B->c_img; a.n = B->c_n;
@@ -442,17 +438,17 @@ static int batch_pose(b200vo_batch* B, const float* lm_obj, const int* n_lm, con
         PoseBatchIO io;
         io.n_lm = n_lm; io.lm_next = lm_next; io.lm_status = lm_status; io.lm_obj = lm_obj;
         io.c_orig = B->c_orig; io.mask_out = inlier_mask; io.n_inl_out = n_inliers; io.ok_out = pnp_ok;
-        VO_TRY(vo_pnp_fused_launch(ctx, a, io));
+        VO_TRY(vo_pnp_fused_launch(ctx, a, io, stream));
     } else {
-        compact_tracked_kernel<<<B->batch, 256, 0, ctx->stream>>>(c.max_landmarks, n_lm, lm_next, lm_status, lm_obj,
-                                                                  B->c_obj, B->c_img, B->c_n, B->c_orig);
+        compact_tracked_kernel<<<B->batch, 256, 0, stream>>>(c.max_landmarks, n_lm, lm_next, lm_status, lm_obj,
+                                                             B->c_obj, B->c_img, B->c_n, B->c_orig);
         ctx->launches++;
-        VO_TRY(vo_pnp_launch(ctx, a, true));
-        scatter_mask_kernel<<<B->batch, 256, 0, ctx->stream>>>(c.max_landmarks, a.ok, a.n_inliers, B->inliers, B->c_orig,
-                                                               inlier_mask, n_inliers, pnp_ok);
+        VO_TRY(vo_pnp_launch(ctx, a, true, stream));
+        scatter_mask_kernel<<<B->batch, 256, 0, stream>>>(c.max_landmarks, a.ok, a.n_inliers, B->inliers, B->c_orig,
+                                                          inlier_mask, n_inliers, pnp_ok);
         ctx->launches++;
     }
-    if (B->prof_row_open) { prof_mark(B, 3); B->prof_n++; B->prof_row_open = false; }
+    if (B->prof_row_open) { prof_mark(B, 3, stream); B->prof_n++; B->prof_row_open = false; }
     VO_CUDA(ctx, cudaGetLastError());
     return 0;
 }
@@ -480,24 +476,23 @@ static int batch_track_pose_overlapped(b200vo_batch* B, const uint8_t* frames_de
 {
     b200vo_ctx* ctx = B->ctx;
     cudaStream_t main_stream = ctx->stream;
-    VO_TRY(batch_track(B, 0, B->batch, frames_dev, lm_pts, n_lm, cand_pts, n_cand, lm_next, lm_status, cand_next, cand_status, 3));
+    VO_TRY(batch_track(B, main_stream, 0, B->batch, frames_dev, lm_pts, n_lm, cand_pts, n_cand, lm_next, lm_status, cand_next,
+                       cand_status, 3));
     VO_CUDA(ctx, cudaEventRecord(B->klt_ev, main_stream));          // pyramids and every input of the step are in place
     VO_CUDA(ctx, cudaStreamWaitEvent(B->pose_stream, B->klt_ev, 0));
-    ctx->stream = B->pose_stream;
-    int rc = batch_track(B, 0, B->batch, frames_dev, lm_pts, n_lm, cand_pts, n_cand, lm_next, lm_status, cand_next, cand_status, 1);
-    if (!rc) rc = (int)cudaEventRecord(B->lm_ev, B->pose_stream);
-    if (!rc && obj_ready) rc = (int)cudaStreamWaitEvent(B->pose_stream, obj_ready, 0);
-    if (!rc) rc = batch_pose(B, lm_obj, n_lm, lm_next, lm_status, pose, pnp_ok, inlier_mask, n_inliers);
-    ctx->stream = main_stream;
-    if (rc) return rc < 0 ? rc : vo_cuda_fail(ctx, (cudaError_t)rc, "pose stream");
+    VO_TRY(batch_track(B, B->pose_stream, 0, B->batch, frames_dev, lm_pts, n_lm, cand_pts, n_cand, lm_next, lm_status, cand_next,
+                       cand_status, 1));
+    VO_CUDA(ctx, cudaEventRecord(B->lm_ev, B->pose_stream));
+    if (obj_ready) VO_CUDA(ctx, cudaStreamWaitEvent(B->pose_stream, obj_ready, 0));
+    VO_TRY(batch_pose(B, B->pose_stream, lm_obj, n_lm, lm_next, lm_status, pose, pnp_ok, inlier_mask, n_inliers));
     VO_CUDA(ctx, cudaEventRecord(B->pose_ev, B->pose_stream));
     // The tracker is a persistent kernel (one grid fills every SM until its queue is empty): launched beside the
     // landmark set, the candidate set would hold half the machine and the landmark tracks -- which the pose chain
     // waits for -- would take twice as long.  So: landmark set alone, then candidate set and pose chain side by side.
-    static const bool serial = getenv("B200VO_POSE_SERIAL") != nullptr;   // A/B switch for measurements: candidate set after the pose chain
-    VO_CUDA(ctx, cudaStreamWaitEvent(main_stream, serial ? B->pose_ev : B->lm_ev, 0));
+    VO_CUDA(ctx, cudaStreamWaitEvent(main_stream, B->lm_ev, 0));
     if (cand_ready) VO_CUDA(ctx, cudaStreamWaitEvent(main_stream, cand_ready, 0));   // candidate keypoints uploaded beside the landmark tracker
-    VO_TRY(batch_track(B, 0, B->batch, frames_dev, lm_pts, n_lm, cand_pts, n_cand, lm_next, lm_status, cand_next, cand_status, 2));
+    VO_TRY(batch_track(B, main_stream, 0, B->batch, frames_dev, lm_pts, n_lm, cand_pts, n_cand, lm_next, lm_status, cand_next,
+                       cand_status, 2));
     VO_CUDA(ctx, cudaEventRecord(B->cand_ev, main_stream));
     VO_CUDA(ctx, cudaStreamWaitEvent(main_stream, B->pose_ev, 0));
     return 0;
@@ -695,7 +690,6 @@ extern "C" int b200vo_batch_step(b200vo_batch* B, const uint8_t* frames, const f
         // The frames go up chunk by chunk, back to back on the copy stream; chunk k's pyramids + landmark tracker
         // run on a compute stream as soon as its frames have landed (the later chunks are on the wire meanwhile);
         // its candidate tracker follows on the ctx stream, and the pose chain starts when the last landmark tracks are in.
-        int rc_chunks = 0;
         if (nchunks > 1) {
             VO_CUDA(ctx, cudaStreamWaitEvent(B->pre_stream, B->step_end_ev, 0));   // B->raw is free again
             VO_CUDA(ctx, cudaStreamWaitEvent(B->pre_stream, B->done_ev, 0));       // behind the step's small uploads
@@ -707,44 +701,38 @@ extern "C" int b200vo_batch_step(b200vo_batch* B, const uint8_t* frames, const f
                 VO_CUDA(ctx, cudaEventRecord(B->copy_ev[k], B->pre_stream));
             }
         }
-        for (int k = 0; k < nchunks && !rc_chunks; ++k) {
+        for (int k = 0; k < nchunks; ++k) {
             const int b0 = k * per, n_here = (b0 + per <= nb ? per : nb - b0);
             if (n_here <= 0) break;
             cudaStream_t cs = nchunks > 1 ? B->chunk_stream[k % B200VO_BATCH_STREAMS] : main_stream;
             if (nchunks > 1) VO_CUDA(ctx, cudaStreamWaitEvent(cs, B->copy_ev[k], 0));
             else VO_CUDA(ctx, cudaMemcpyAsync(B->raw.p, fsrc, (size_t)n_here * fb, cudaMemcpyHostToDevice, cs));
-            ctx->stream = cs;   // the launch helpers enqueue on ctx->stream
-            rc_chunks = batch_track(B, b0, n_here, (const uint8_t*)B->raw.p, (const float*)(di + o_lmp), (const int*)(di + o_nlm),
-                                    (const float*)(di + o_cp), (const int*)(di + o_nc), (float*)(dq + q_lmn), dq + q_lms,
-                                    (float*)(dq + q_cn), dq + q_cs, 4);
-            ctx->stream = main_stream;
-            if (!rc_chunks && nchunks > 1) {
+            VO_TRY(batch_track(B, cs, b0, n_here, (const uint8_t*)B->raw.p, (const float*)(di + o_lmp), (const int*)(di + o_nlm),
+                               (const float*)(di + o_cp), (const int*)(di + o_nc), (float*)(dq + q_lmn), dq + q_lms,
+                               (float*)(dq + q_cn), dq + q_cs, 4));
+            if (nchunks > 1) {
                 VO_CUDA(ctx, cudaEventRecord(B->chunk_ev[k], cs));
                 // this chunk's candidates follow on the (normal-priority) ctx stream: they fill the SMs whenever the
                 // landmark trackers of later chunks are still waiting for their frames
                 VO_CUDA(ctx, cudaStreamWaitEvent(main_stream, B->chunk_ev[k], 0));
                 VO_CUDA(ctx, cudaStreamWaitEvent(B->pose_stream, B->chunk_ev[k], 0));
-                rc_chunks = batch_track(B, b0, n_here, nullptr, (const float*)(di + o_lmp), (const int*)(di + o_nlm),
-                                        (const float*)(di + o_cp), (const int*)(di + o_nc), (float*)(dq + q_lmn), dq + q_lms,
-                                        (float*)(dq + q_cn), dq + q_cs, 2);
+                VO_TRY(batch_track(B, main_stream, b0, n_here, nullptr, (const float*)(di + o_lmp), (const int*)(di + o_nlm),
+                                   (const float*)(di + o_cp), (const int*)(di + o_nc), (float*)(dq + q_lmn), dq + q_lms,
+                                   (float*)(dq + q_cn), dq + q_cs, 2));
             }
         }
-        if (rc_chunks) return rc_chunks;
         if (nchunks == 1) {
             VO_CUDA(ctx, cudaEventRecord(B->lm_ev, main_stream));
             VO_CUDA(ctx, cudaStreamWaitEvent(B->pose_stream, B->lm_ev, 0));
-            VO_TRY(batch_track(B, 0, nb, nullptr, (const float*)(di + o_lmp), (const int*)(di + o_nlm), (const float*)(di + o_cp),
+            VO_TRY(batch_track(B, main_stream, 0, nb, nullptr, (const float*)(di + o_lmp), (const int*)(di + o_nlm), (const float*)(di + o_cp),
                                (const int*)(di + o_nc), (float*)(dq + q_lmn), dq + q_lms, (float*)(dq + q_cn), dq + q_cs, 2));
         }
         VO_CUDA(ctx, cudaEventRecord(B->cand_ev, main_stream));
         // the pose chain (high priority) starts once every chunk's landmark tracks are done
         if (!packed) VO_CUDA(ctx, cudaStreamWaitEvent(B->pose_stream, B->obj_ev, 0));
         VO_CUDA(ctx, cudaEventRecord(B->lm_ev, B->pose_stream));
-        ctx->stream = B->pose_stream;
-        const int rc_pose = batch_pose(B, (const float*)(di + o_lmo), (const int*)(di + o_nlm), (const float*)(dq + q_lmn), dq + q_lms,
-                                       (double*)(dq + q_pose), dq + q_ok, dq + q_mask, (int*)(dq + q_ni));
-        ctx->stream = main_stream;
-        if (rc_pose) return rc_pose;
+        VO_TRY(batch_pose(B, B->pose_stream, (const float*)(di + o_lmo), (const int*)(di + o_nlm), (const float*)(dq + q_lmn),
+                          dq + q_lms, (double*)(dq + q_pose), dq + q_ok, dq + q_mask, (int*)(dq + q_ni)));
         VO_CUDA(ctx, cudaEventRecord(B->pose_ev, B->pose_stream));
         VO_CUDA(ctx, cudaStreamWaitEvent(main_stream, B->pose_ev, 0));
     }

@@ -46,7 +46,7 @@ static int upload_into_slot(b200vo_ctx* ctx, int slot, int stage_idx, const uint
     else for (int y = 0; y < rows; ++y) memcpy(hp + (size_t)y * cols, img + (size_t)y * step, (size_t)cols);
     VO_CUDA(ctx, cudaMemcpyAsync(ctx->d_stage_img[stage_idx].p, hp, raw_bytes, cudaMemcpyHostToDevice, ctx->stream));
     VO_TRY(vo_build_pyramids(ctx, (const uint8_t*)ctx->d_stage_img[stage_idx].p, raw_bytes, rows, cols, g,
-                             (uint8_t*)fs.slab.p, g.slab_bytes, 1));
+                             (uint8_t*)fs.slab.p, g.slab_bytes, 1, ctx->stream));
     fs.geom = g;
     fs.rows = rows;
     fs.cols = cols;
@@ -80,8 +80,8 @@ static int klt_on_slots(b200vo_ctx* ctx, int prev_slot, int next_slot, const flo
     uint8_t* hp = (uint8_t*)ctx->h_pin + pin_off;
     memcpy(hp, prev_pts, (size_t)n * 8);
     VO_CUDA(ctx, cudaMemcpyAsync(d_pts, hp, (size_t)n * 8, cudaMemcpyHostToDevice, ctx->stream));
-    VO_TRY(vo_klt_launch(ctx, g, (const uint8_t*)fp.slab.p, 0, (const uint8_t*)fn.slab.p, 0, 1, n, nullptr, n,
-                         d_pts, d_next, d_st, d_err, kp));
+    const KltPointSet set{n, nullptr, d_pts, d_next, d_st, d_err};
+    VO_TRY(vo_klt_launch2(ctx, g, (const uint8_t*)fp.slab.p, 0, (const uint8_t*)fn.slab.p, 0, 1, &set, 1, n, kp, ctx->stream));
     // one D2H of next|err|status (contiguous on the device)
     VO_CUDA(ctx, cudaMemcpyAsync(hp + b_pts, d_next, b_pts + b_err + b_st, cudaMemcpyDeviceToHost, ctx->stream));
     VO_CUDA(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
@@ -132,7 +132,7 @@ static int build_slot_from_device(b200vo_ctx* ctx, int slot, int stage_idx, cons
                                        cudaMemcpyDeviceToDevice, ctx->stream));
         raw = (const uint8_t*)ctx->d_stage_img[stage_idx].p;
     }
-    VO_TRY(vo_build_pyramids(ctx, raw, raw_bytes, rows, cols, g, (uint8_t*)fs.slab.p, g.slab_bytes, 1));
+    VO_TRY(vo_build_pyramids(ctx, raw, raw_bytes, rows, cols, g, (uint8_t*)fs.slab.p, g.slab_bytes, 1, ctx->stream));
     fs.geom = g; fs.rows = rows; fs.cols = cols; fs.valid = true;
     return 0;
 }
@@ -157,8 +157,9 @@ extern "C" int b200vo_calc_optical_flow_pyr_lk_dev(b200vo_ctx* ctx, const uint8_
     VO_TRY(build_slot_from_device(ctx, s1, 1, next_dev, rows, cols, next_step, win_w, win_h, max_level));
     const KltParams kp = make_params(win_w, win_h, crit_type, crit_max_count, crit_eps, min_eig_thr);
     const FrameSlot& fp = ctx->slots[s0];
-    return vo_klt_launch(ctx, fp.geom, (const uint8_t*)fp.slab.p, 0, (const uint8_t*)ctx->slots[s1].slab.p, 0, 1, n, nullptr, n,
-                         prev_pts_dev, next_pts_dev, status_dev, err_dev, kp);
+    const KltPointSet set{n, nullptr, prev_pts_dev, next_pts_dev, status_dev, err_dev};
+    return vo_klt_launch2(ctx, fp.geom, (const uint8_t*)fp.slab.p, 0, (const uint8_t*)ctx->slots[s1].slab.p, 0, 1, &set, 1, n, kp,
+                          ctx->stream);
 }
 
 extern "C" int b200vo_frame_upload(b200vo_ctx* ctx, int slot, const uint8_t* img, int rows, int cols,

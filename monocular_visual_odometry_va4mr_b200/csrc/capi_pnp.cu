@@ -50,7 +50,7 @@ static int pnp_run(b200vo_ctx* ctx, const float* obj, const float* img, int n, c
         memcpy(hs, samples, (size_t)iters * 16);
         VO_CUDA(ctx, cudaMemcpyAsync(a.samples, hs, (size_t)iters * 16, cudaMemcpyHostToDevice, ctx->stream));
     }
-    VO_TRY(vo_pnp_launch(ctx, a, samples == nullptr));
+    VO_TRY(vo_pnp_launch(ctx, a, samples == nullptr, ctx->stream));
     uint8_t* ho = hp + in_bytes;
     VO_CUDA(ctx, cudaMemcpyAsync(ho, dout, out_bytes, cudaMemcpyDeviceToHost, ctx->stream));
     int* hsmall = (int*)(ho + out_bytes);
@@ -132,7 +132,7 @@ extern "C" int b200vo_solve_pnp_ransac_p3p_dev(b200vo_ctx* ctx, const float* obj
     a.inliers = inliers_dev; a.pose = pose_dev; a.ok = success_dev;
     vo_pnp_carve_workspace(a, d + 256 + b_mask);
     VO_CUDA(ctx, cudaMemcpyAsync(d, &n, sizeof(int), cudaMemcpyHostToDevice, ctx->stream));   // pageable source: staged before the call returns
-    VO_TRY(vo_pnp_launch(ctx, a, true));
+    VO_TRY(vo_pnp_launch(ctx, a, true, ctx->stream));
     pnp_export_kernel<<<1, 1, 0, ctx->stream>>>(a.n_inliers, a.ok, n_inliers_dev);
     ctx->launches++;
     VO_CUDA(ctx, cudaGetLastError());
@@ -164,7 +164,7 @@ extern "C" int b200vo_debug_pose_phases(b200vo_ctx* ctx, const float* obj_dev, c
     VO_CUDA(ctx, cudaMemcpyAsync(d, &n, sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
     if (!vo_pnp_fused_ok(a, true)) return vo_set_err(ctx, B200VO_E_UNSUPPORTED, "the fused pose kernel is not in use for this size");
     VO_CUDA(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
-    VO_TRY(vo_pnp_launch(ctx, a, true));
+    VO_TRY(vo_pnp_launch(ctx, a, true, ctx->stream));
     VO_CUDA(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
     VO_CUDA(ctx, cudaMemcpyAsync(clk_host, a.phase_clk, 16 * sizeof(long long), cudaMemcpyDeviceToHost, ctx->stream));
     VO_CUDA(ctx, cudaStreamSynchronize(ctx->stream));

@@ -570,7 +570,7 @@ extern "C" int b200vo_good_features_to_track(b200vo_ctx* ctx, const uint8_t* img
     if (step == (size_t)cols) memcpy(hp, img, npx);
     else for (int y = 0; y < rows; ++y) memcpy(hp + (size_t)y * cols, img + (size_t)y * step, (size_t)cols);
     VO_CUDA(ctx, cudaMemcpyAsync(ctx->d_stage_img[1].p, hp, npx, cudaMemcpyHostToDevice, ctx->stream));
-    VO_TRY(vo_build_pyramids(ctx, (const uint8_t*)ctx->d_stage_img[1].p, npx, rows, cols, g, (uint8_t*)fs.slab.p, g.slab_bytes, 1));
+    VO_TRY(vo_build_pyramids(ctx, (const uint8_t*)ctx->d_stage_img[1].p, npx, rows, cols, g, (uint8_t*)fs.slab.p, g.slab_bytes, 1, ctx->stream));
     const uint8_t* d_img = (const uint8_t*)fs.slab.p + g.off[0];
     // scratch: cov | eig | keys | sorted | cells | small
     const int cell = min_dist >= 1 ? (int)llrint(min_dist) : 1;
@@ -746,7 +746,7 @@ extern "C" int b200vo_good_features_to_track_dev(b200vo_ctx* ctx, const uint8_t*
                                        cudaMemcpyDeviceToDevice, ctx->stream));
         raw = (const uint8_t*)ctx->d_stage_img[1].p;
     }
-    VO_TRY(vo_build_pyramids(ctx, raw, npx, rows, cols, g, (uint8_t*)fs.slab.p, g.slab_bytes, 1));
+    VO_TRY(vo_build_pyramids(ctx, raw, npx, rows, cols, g, (uint8_t*)fs.slab.p, g.slab_bytes, 1, ctx->stream));
     VO_TRY(vo_reserve(ctx, ctx->d_scratch[2], vo_gftt_batch_workspace(rows, cols, 1, max_corners > 0 ? max_corners : 1)));
     float* d_out = nullptr;
     int* d_small = nullptr;

@@ -98,7 +98,7 @@ void vo_pyr_geom(int rows, int cols, int levels, PyrGeom* g);
 Pyramid vo_pyramid_at(const PyrGeom& g, uint8_t* slab);
 // raw (tight, device) -> bordered level 0, then levels 1..L-1; `batch` slabs/raws strided.
 int vo_build_pyramids(b200vo_ctx* ctx, const uint8_t* d_raw, size_t raw_stride, int rows, int cols,
-                      const PyrGeom& g, uint8_t* d_slab, size_t slab_stride, int batch);
+                      const PyrGeom& g, uint8_t* d_slab, size_t slab_stride, int batch, cudaStream_t stream);
 
 // ---- gftt.cu: detection on device-resident bordered level-0 images, one per batch entry ----
 #define VO_GFTT_SMALL 4          // ints per image in the result block: max bits | n candidates | n corners | spare
@@ -117,12 +117,7 @@ struct KltPointSet {
     float* err;         // [batch][cap] or nullptr
 };
 void vo_klt_trace_read(b200vo_ctx* ctx, std::vector<unsigned long long>& out);   // B200VO_TRACE_FILE aid
+// Tracks the points of up to two sets in `batch` independent frame pairs, on `stream`.
 int vo_klt_launch2(b200vo_ctx* ctx, const PyrGeom& g, const uint8_t* d_prev_slab, size_t prev_stride,
                    const uint8_t* d_next_slab, size_t next_stride, int batch, const KltPointSet* sets, int n_sets,
-                   int n_fixed, const KltParams& kp);
-// Tracks points of `batch` independent frame pairs.  pts/next/status/err are
-// [batch][cap] arrays; n_pts (device) gives the live count per pair (or nullptr -> n_fixed).
-int vo_klt_launch(b200vo_ctx* ctx, const PyrGeom& g, const uint8_t* d_prev_slab, size_t prev_stride,
-                  const uint8_t* d_next_slab, size_t next_stride, int batch, int cap,
-                  const int* d_n_pts, int n_fixed, const float* d_pts, float* d_next,
-                  uint8_t* d_status, float* d_err, const KltParams& kp);
+                   int n_fixed, const KltParams& kp, cudaStream_t stream);

@@ -257,7 +257,6 @@ klt_kernel(const KltArgs a)
     }
 }
 
-#include "klt_v2.cuh"
 #include "klt_v3.cuh"
 
 #define KLT_QUEUE_SLOTS 1024
@@ -265,7 +264,7 @@ klt_kernel(const KltArgs a)
 
 int vo_klt_launch2(b200vo_ctx* ctx, const PyrGeom& g, const uint8_t* d_prev_slab, size_t prev_stride,
                    const uint8_t* d_next_slab, size_t next_stride, int batch, const KltPointSet* sets, int n_sets,
-                   int n_fixed, const KltParams& kp)
+                   int n_fixed, const KltParams& kp, cudaStream_t stream)
 {
     if (batch <= 0 || n_sets <= 0) return 0;
     KltArgs a{};
@@ -298,20 +297,19 @@ int vo_klt_launch2(b200vo_ctx* ctx, const PyrGeom& g, const uint8_t* d_prev_slab
     size_t smem = (size_t)a.smem_per_warp * KLT_WARPS;
     const long long total_warps = (long long)batch * (a.cap[0] + a.cap[1]);
     const unsigned grid = (unsigned)((total_warps + KLT_WARPS - 1) / KLT_WARPS);
-    void (*kern)(const KltArgs) = nullptr;
-    // v3 = persistent warps + work queue (default); B200VO_KLT=v2 keeps the one-warp-per-slot kernel for A/B runs
-    static const bool use_v2 = getenv("B200VO_KLT") && !strcmp(getenv("B200VO_KLT"), "v2");
+    void (*kern)(const KltArgs) = klt_kernel<0, 0>;
+    // the staged kernel (persistent warps + work queue) for the two window sizes it is built for; the queue counter is
+    // an int, so a launch of 2^30 features or more takes the generic kernel (same arithmetic, same results)
     const bool sized = (kp.win_w == 21 && kp.win_h == 21) || (kp.win_w == 15 && kp.win_h == 15);
-    const bool v3 = sized && !use_v2 && total_warps < (1ll << 30);
     unsigned launch_grid = grid;
-    int min_ctas = 0;
-    if (v3) {
+    if (sized && total_warps < (1ll << 30)) {
+        int min_ctas;
         if (kp.win_w == 21) { kern = klt_kernel_v3<21, 21>; smem = (size_t)KV3<21, 21>::PER_WARP * KLT_WARPS + 64; min_ctas = KV3<21, 21>::MIN_CTAS; }
         else { kern = klt_kernel_v3<15, 15>; smem = (size_t)KV3<15, 15>::PER_WARP * KLT_WARPS + 64; min_ctas = KV3<15, 15>::MIN_CTAS; }
         if (!ctx->d_klt_queue.p) {
             VO_TRY(vo_reserve(ctx, ctx->d_klt_queue, (size_t)KLT_QUEUE_SLOTS * KLT_QUEUE_INTS * sizeof(int)));
-            VO_CUDA(ctx, cudaMemsetAsync(ctx->d_klt_queue.p, 0, (size_t)KLT_QUEUE_SLOTS * KLT_QUEUE_INTS * sizeof(int), ctx->stream));
-            VO_CUDA(ctx, cudaStreamSynchronize(ctx->stream));   // other streams of this context launch trackers too
+            VO_CUDA(ctx, cudaMemsetAsync(ctx->d_klt_queue.p, 0, (size_t)KLT_QUEUE_SLOTS * KLT_QUEUE_INTS * sizeof(int), stream));
+            VO_CUDA(ctx, cudaStreamSynchronize(stream));   // other streams of this context launch trackers too
         }
         // a ring of counters: launches that run concurrently (landmark / candidate sets, chunk streams) never share one,
         // and each kernel re-arms its own slot when its last warp retires
@@ -319,9 +317,6 @@ int vo_klt_launch2(b200vo_ctx* ctx, const PyrGeom& g, const uint8_t* d_prev_slab
         const unsigned resident = (unsigned)(ctx->num_sms * min_ctas);
         launch_grid = grid < resident ? grid : resident;
     }
-    else if (kp.win_w == 21 && kp.win_h == 21) { kern = klt_kernel_v2<21, 21>; smem = (size_t)KV2<21, 21>::PER_WARP * KLT_WARPS + 64; }
-    else if (kp.win_w == 15 && kp.win_h == 15) { kern = klt_kernel_v2<15, 15>; smem = (size_t)KV2<15, 15>::PER_WARP * KLT_WARPS + 64; }
-    else kern = klt_kernel<0, 0>;
     {   // function attributes: once per kernel and process (the calls cost microseconds each on the launch path)
         static void* configured[8] = {};
         bool seen = false;
@@ -335,7 +330,7 @@ int vo_klt_launch2(b200vo_ctx* ctx, const PyrGeom& g, const uint8_t* d_prev_slab
             if (free_slot >= 0 && kern != klt_kernel<0, 0>) configured[free_slot] = (void*)kern;   // the generic kernel's smem size varies per call
         }
     }
-    kern<<<launch_grid, KLT_WARPS * 32, smem, ctx->stream>>>(a);
+    kern<<<launch_grid, KLT_WARPS * 32, smem, stream>>>(a);
     ctx->launches++;
     VO_CUDA(ctx, cudaGetLastError());
     return 0;
@@ -349,13 +344,4 @@ void vo_klt_trace_read(b200vo_ctx* ctx, std::vector<unsigned long long>& out)
     std::vector<unsigned long long> raw((size_t)KLT_QUEUE_SLOTS * KLT_QUEUE_INTS / 2);
     if (cudaMemcpy(raw.data(), ctx->d_klt_queue.p, raw.size() * 8, cudaMemcpyDeviceToHost) != cudaSuccess) return;
     for (int s = 0; s < KLT_QUEUE_SLOTS; ++s) { out.push_back(raw[(size_t)s * 4 + 1]); out.push_back(raw[(size_t)s * 4 + 2]); }
-}
-
-int vo_klt_launch(b200vo_ctx* ctx, const PyrGeom& g, const uint8_t* d_prev_slab, size_t prev_stride,
-                  const uint8_t* d_next_slab, size_t next_stride, int batch, int cap,
-                  const int* d_n_pts, int n_fixed, const float* d_pts, float* d_next,
-                  uint8_t* d_status, float* d_err, const KltParams& kp)
-{
-    KltPointSet s{cap, d_n_pts, d_pts, d_next, d_status, d_err};
-    return vo_klt_launch2(ctx, g, d_prev_slab, prev_stride, d_next_slab, next_stride, batch, &s, 1, n_fixed, kp);
 }

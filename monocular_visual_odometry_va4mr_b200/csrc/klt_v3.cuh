@@ -1,20 +1,56 @@
-// klt_kernel_v3<WW,WH>: klt_kernel_v2 (same arithmetic, bit-identical results) reworked around the
-// round-2 source-level capture (profiles/r2a_klt_source_hot.txt):
+// klt_kernel_v3<WW,WH>: the tracker for the two window sizes the workloads use (15x15: the reference's
+// options, main.py:36; 21x21: cv2's default).  Same arithmetic as klt_kernel, bit-identical results:
+//   * a lane owns a run of 8 horizontally adjacent window pixels (row y, x0 = 0, 8, 16) instead of every
+//     32nd pixel, read with two LDS.64 per row from rows of 40 bytes (5 eight-byte slots) and re-aligned
+//     with funnel shifts: with lanes 0-15 on the left runs and lanes 16-31 on the right runs each half-warp
+//     touches 15 distinct slots, so the window reads are conflict-free;
+//   * the bilinear interpolation I00*w00 + I01*w01 (+ next row) is two dp2a (16-bit weights x 8-bit pixels)
+//     instead of four IMAD; the Scharr derivative of the previous image is 5 dp4a per pixel on the staged patch;
+//   * the window of the NEXT image is staged in shared memory per level by 8-byte cp.async (window + 4 px
+//     margin, restaged only if the point leaves it), so iterations never touch L1/L2;
+//   * the template gradients live in registers; sum(Iwin*dI) is folded into two constants, so an iteration
+//     needs neither Iwin nor a subtraction per pixel;
 //   * PERSISTENT warps + an atomic work queue (SURVEY 7.3): a warp fetches the next feature when its own
-//     converges, so a CTA slot is never held by the slowest of four features (warps active 6.7 of 8 before),
-//     and small shards (8 sequences per GPU in the strong-scaling run) are no longer tail-bound;
+//     converges, so a CTA slot is never held by the slowest of four features, and small shards (8 sequences
+//     per GPU in the strong-scaling run) are not tail-bound (profiles/r2a_klt_source_hot.txt);
 //   * iteration loop: the staged-window test and the image-range test are ONE unsigned compare per axis
 //     against bounds fixed at staging time; plain F2I.FLOOR instead of the guarded cvFloor (positions are
 //     finite inside the loop, the guard stays at the level entry); the two exact 64-bit warp sums take a
 //     single-REDUX fast path whenever no lane partial can overflow int32 (a vote decides; the hi/lo split
-//     path is kept for the rest); packed weights by one IMAD each;
-//   * every 8-pixel run is read with two LDS.64 per row from rows of 40 bytes (5 eight-byte slots): with
-//     lanes 0-15 on the left runs and lanes 16-31 on the right runs each half-warp touches 15 distinct slots,
-//     so the window reads are conflict-free (v2: 3 LDS.32 per row, always a 2-way conflict between lane 29
-//     and lane 0 -- any odd word stride has one);
-//   * staging by 8-byte cp.async (5 per row instead of 9): half the LDGSTS and address arithmetic per level.
+//     path is kept for the rest); packed weights by one IMAD each.
 #pragma once
 #include <type_traits>
+
+// 16-bit weights x 8-bit pixels.  The weights are SIGNED halves: iw11 = 2^14 - iw00 - iw01 - iw10 is -1
+// when the three rounded weights add up to 2^14 + 1 (a fractional part of ~0 in x or y, about one
+// position in a thousand) -- cv2 carries that -1 through its integer arithmetic, and so must this.
+__device__ __forceinline__ uint32_t dp2a_lo_u(uint32_t a, uint32_t b, uint32_t c)
+{
+    int d;
+    asm("dp2a.lo.s32.u32 %0, %1, %2, %3;" : "=r"(d) : "r"(a), "r"(b), "r"((int)c));
+    return (uint32_t)d;
+}
+__device__ __forceinline__ uint32_t dp2a_hi_u(uint32_t a, uint32_t b, uint32_t c)
+{
+    int d;
+    asm("dp2a.hi.s32.u32 %0, %1, %2, %3;" : "=r"(d) : "r"(a), "r"(b), "r"((int)c));
+    return (uint32_t)d;
+}
+__device__ __forceinline__ int dp4a_us(uint32_t a, int b, int c)   // unsigned pixels x signed coefficients
+{
+    int d;
+    asm("dp4a.u32.s32 %0, %1, %2, %3;" : "=r"(d) : "r"(a), "r"(b), "r"(c));
+    return d;
+}
+
+// asynchronous global -> shared staging (LDGSTS): the copy proceeds while the warp computes
+__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
+__device__ __forceinline__ void cp_async_wait_pending(int n)   // wait until at most n groups are pending
+{
+    if (n <= 0) asm volatile("cp.async.wait_group 0;" ::: "memory");
+    else if (n == 1) asm volatile("cp.async.wait_group 1;" ::: "memory");
+    else asm volatile("cp.async.wait_group 2;" ::: "memory");
+}
 
 template <int WW, int WH>
 struct KV3 {

@@ -8,23 +8,20 @@
 // first) and the ratio decision are bit-exact with cv2.
 //
 // The contraction runs on the 5th-gen tensor cores: tcgen05.mma (cta_group::1, kind::f16,
-// M=128, N=256, K=16 x 8) issued by one thread, operands staged by TMA into 128B-swizzled
-// shared memory, accumulators double-buffered in TMEM (2 x 256 columns).  Sixteen epilogue warps
-// (four per TMEM lane quadrant) pull the accumulators with tcgen05.ld and keep a running (best, second) per query row in
-// registers -- the Q x T distance matrix is never materialised.  A CTA owns one 128-query tile and
-// a contiguous range of train tiles; partial top-2s of the ranges are merged in index order.
+// M=128, N=128, K=16 x 9) issued by one thread, operands staged by TMA into swizzled shared
+// memory, accumulators double-buffered in TMEM (2 stages x 2 query halves x 128 columns).  Sixteen
+// epilogue warps (four per TMEM lane quadrant) pull the accumulators with tcgen05.ld and keep a running
+// (best, second) per query row in registers -- the Q x T distance matrix is never materialised.  A CTA
+// owns a contiguous run of (query pair, train tile) units; partial top-2s of the runs are merged in
+// index order.
 #include "internal.cuh"
 #include "tma.cuh"
 #include <cuda_fp16.h>
 
 #define KNN_BM 128
-#define KNN_BN 256
 #define KNN_DIM 128
 #define KNN_EPI_WARPS 16
 #define KNN_THREADS (64 + 32 * KNN_EPI_WARPS)
-#define KNN_A_BYTES (KNN_BM * KNN_DIM * 2)        // 32 KB
-#define KNN_B_BYTES (KNN_BN * KNN_DIM * 2)        // 64 KB per stage
-#define KNN_SMEM (1024 + KNN_A_BYTES + 2 * KNN_B_BYTES + 2 * KNN_BN * 4 + 256 + KNN_BM * 4 * 4)   // barriers live in the first 128 B of the 256-B block
 #define KNN_BIG 3.0e38f
 
 // ------------------------------------------------------------------ PTX wrappers (TMA/mbarrier: tma.cuh)
@@ -42,19 +39,6 @@ __device__ __forceinline__ void tc_mma_f16(uint32_t d_tmem, uint64_t adesc, uint
         "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
         ::"r"(d_tmem), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
 }
-__device__ __forceinline__ void tc_ld32(uint32_t taddr, uint32_t* v)
-{
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-        "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-        "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-        : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]),
-          "=r"(v[8]), "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15]),
-          "=r"(v[16]), "=r"(v[17]), "=r"(v[18]), "=r"(v[19]), "=r"(v[20]), "=r"(v[21]), "=r"(v[22]), "=r"(v[23]),
-          "=r"(v[24]), "=r"(v[25]), "=r"(v[26]), "=r"(v[27]), "=r"(v[28]), "=r"(v[29]), "=r"(v[30]), "=r"(v[31])
-        : "r"(taddr) : "memory");
-}
-__device__ __forceinline__ void tc_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 
 // K-major, 128B-swizzled operand tile: rows of 128 B, 8-row groups 1024 B apart
 __device__ __forceinline__ uint64_t umma_desc_sw128(uint32_t smem_addr)
@@ -62,205 +46,14 @@ __device__ __forceinline__ uint64_t umma_desc_sw128(uint32_t smem_addr)
     return (uint64_t)((smem_addr >> 4) & 0x3FFF) | (1ull << 16) | (64ull << 32) | (1ull << 46) | (2ull << 61);
 }
 
-// ------------------------------------------------------------------ prep: f32 -> fp16 + norms
-__global__ void __launch_bounds__(256)
-knn_prep_kernel(const float* __restrict__ src, int n, int n_pad, __half* __restrict__ dst, float* __restrict__ norm,
-                float pad_norm, int* __restrict__ bad)
-{
-    const int row = blockIdx.x * 8 + (threadIdx.x >> 5);
-    const int lane = threadIdx.x & 31;
-    if (row >= n_pad) return;
-    float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-    if (row < n) v = reinterpret_cast<const float4*>(src + (size_t)row * KNN_DIM)[lane];
-    const float a[4] = {v.x, v.y, v.z, v.w};
-    float s = 0.f;
-    bool ok = true;
-#pragma unroll
-    for (int k = 0; k < 4; ++k) {
-        ok = ok && (a[k] >= 0.f) && (a[k] <= 255.f) && (a[k] == floorf(a[k]));
-        s += a[k] * a[k];
-    }
-    __half2 h0 = __floats2half2_rn(a[0], a[1]), h1 = __floats2half2_rn(a[2], a[3]);
-    uint2 pk;
-    pk.x = *reinterpret_cast<uint32_t*>(&h0);
-    pk.y = *reinterpret_cast<uint32_t*>(&h1);
-    reinterpret_cast<uint2*>(dst + (size_t)row * KNN_DIM)[lane] = pk;
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);   // exact: integers < 2^24
-    if (!__all_sync(0xffffffffu, ok) && lane == 0) atomicOr(bad, 1);
-    if (lane == 0) norm[row] = row < n ? s : pad_norm;
-}
-
-// ------------------------------------------------------------------ GEMM + fused top-2
 struct KnnPartial { float d1, d2; int i1, i2; };
 
-__global__ void __launch_bounds__(KNN_THREADS, 1)
-knn_gemm_top2_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_t,
-                     const float* __restrict__ qnorm, const float* __restrict__ tnorm, int n_tiles_total,
-                     int tiles_per_split, KnnPartial* __restrict__ partial, int nq_pad)
-{
-    extern __shared__ uint8_t smem_raw[];
-    const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
-    const uint32_t sA = base;
-    const uint32_t sB = base + KNN_A_BYTES;
-    const uint32_t sTn = sB + 2 * KNN_B_BYTES;
-    const uint32_t sBar = sTn + 2 * KNN_BN * 4;
-    float* tn_s = reinterpret_cast<float*>(smem_raw + (sTn - smem_u32(smem_raw)));
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(smem_raw + (sBar + 128 - smem_u32(smem_raw)));
-    float* tau_s = reinterpret_cast<float*>(smem_raw + (sBar + 256 - smem_u32(smem_raw)));   // [128 rows][4 column groups]
-    const uint32_t bar_a = sBar, bar_bfull = sBar + 8, bar_bempty = sBar + 24, bar_accfull = sBar + 40, bar_accempty = sBar + 56;
-
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int m0 = blockIdx.x * KNN_BM;
-    const int t0 = blockIdx.y * tiles_per_split;
-    const int t1 = min(t0 + tiles_per_split, n_tiles_total);
-    const int nt = t1 - t0;
-
-    if (threadIdx.x == 0) {
-        mbar_init(bar_a, 1);
-        for (int s = 0; s < 2; ++s) {
-            mbar_init(bar_bfull + 8 * s, 1);
-            mbar_init(bar_bempty + 8 * s, 1);
-            mbar_init(bar_accfull + 8 * s, 1);
-            mbar_init(bar_accempty + 8 * s, 32 * KNN_EPI_WARPS);
-        }
-        mbar_fence_init();
-    }
-    if (warp == 1) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 512;" ::"r"(smem_u32(tmem_slot)) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem_base = *tmem_slot;
-
-    if (warp == 0) {
-        if (lane == 0) {
-            // query tile: two 64-element K blocks, resident for the whole CTA
-            mbar_expect_tx(bar_a, KNN_A_BYTES);
-            tma_load_2d(sA, &map_q, 0, m0, bar_a);
-            tma_load_2d(sA + KNN_A_BYTES / 2, &map_q, 64, m0, bar_a);
-            for (int i = 0; i < nt; ++i) {
-                const int s = i & 1, ph = (i >> 1) & 1;
-                mbar_wait(bar_bempty + 8 * s, ph ^ 1);
-                mbar_expect_tx(bar_bfull + 8 * s, KNN_B_BYTES);
-                const uint32_t dst = sB + s * KNN_B_BYTES;
-                tma_load_2d(dst, &map_t, 0, (t0 + i) * KNN_BN, bar_bfull + 8 * s);
-                tma_load_2d(dst + KNN_B_BYTES / 2, &map_t, 64, (t0 + i) * KNN_BN, bar_bfull + 8 * s);
-            }
-        }
-    } else if (warp == 1) {
-        if (lane == 0) {
-            // instruction descriptor: D=F32, A=B=F16, K-major both, N=256, M=128
-            const uint32_t idesc = (1u << 4) | ((uint32_t)(KNN_BN >> 3) << 17) | ((uint32_t)(KNN_BM >> 4) << 24);
-            mbar_wait(bar_a, 0);
-            for (int i = 0; i < nt; ++i) {
-                const int s = i & 1, ph = (i >> 1) & 1;
-                mbar_wait(bar_accempty + 8 * s, ph ^ 1);
-                mbar_wait(bar_bfull + 8 * s, ph);
-                tc_fence_after();
-                const uint32_t d_tmem = tmem_base + (uint32_t)(s * KNN_BN);
-#pragma unroll
-                for (int kb = 0; kb < 2; ++kb) {
-                    const uint64_t adesc = umma_desc_sw128(sA + kb * (KNN_A_BYTES / 2));
-                    const uint64_t bdesc = umma_desc_sw128(sB + s * KNN_B_BYTES + kb * (KNN_B_BYTES / 2));
-#pragma unroll
-                    for (int k = 0; k < 4; ++k)   // 16 fp16 = 32 B per UMMA_K step inside the swizzle atom
-                        tc_mma_f16(d_tmem, adesc + 2 * k, bdesc + 2 * k, idesc, (kb | k) != 0);
-                }
-                tc_commit(bar_bempty + 8 * s);     // smem stage free once these MMAs have read it
-                tc_commit(bar_accfull + 8 * s);    // accumulator ready for the epilogue
-            }
-        }
-    } else {
-        // epilogue: warp w may touch TMEM lanes 32*(w%4) .. +31; four warps per lane quadrant, each
-        // scanning one 64-column group of every accumulator tile; one query row per thread.
-        const int q = warp & 3;
-        const int sub = (warp - 2) >> 2;          // column group 0..3
-        const int rl = q * 32 + lane;             // row inside the tile
-        const int row = m0 + rl;
-        const int et = (warp - 2) * 32 + lane;    // 0..511
-        // ordering uses d' = |t|^2 - 2 q.t (|q|^2 is constant per row and added at the end); exact integers in fp32
-        float b1 = KNN_BIG, b2 = KNN_BIG;
-        int i1 = -1, i2 = -1;
-        if (et < KNN_BN && nt > 0) tn_s[et] = tnorm[t0 * KNN_BN + et];
-        tau_s[rl * 4 + sub] = KNN_BIG;
-        for (int i = 0; i < nt; ++i) {
-            const int s = i & 1, ph = (i >> 1) & 1;
-            const int j0 = (t0 + i) * KNN_BN;
-            float tn_next = 0.f;
-            const bool pre = et < KNN_BN && i + 1 < nt;
-            if (pre) tn_next = tnorm[j0 + KNN_BN + et];        // in flight while this tile is scanned
-            asm volatile("bar.sync 1, 512;" ::: "memory");
-            {   // the four warps of a row share their running second-best: anything strictly above the
-                // smallest of them cannot enter the global top-2 (entries lowered this way carry index -1)
-                const float4 t4 = *reinterpret_cast<const float4*>(tau_s + rl * 4);
-                const float tau = fminf(fminf(t4.x, t4.y), fminf(t4.z, t4.w)) + 1.0f;   // integers: next value up
-                if (tau < b2) { b2 = tau; i2 = -1; }
-            }
-            mbar_wait(bar_accfull + 8 * s, ph);
-            tc_fence_after();
-            const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(s * KNN_BN + sub * 64);
-#pragma unroll 1
-            for (int c = 0; c < 2; ++c) {
-                uint32_t v[32];
-                tc_ld32(taddr + c * 32, v);
-                tc_ld_wait();
-                const float4* tn4 = reinterpret_cast<const float4*>(tn_s + s * KNN_BN + sub * 64 + c * 32);
-                const int jc = j0 + sub * 64 + c * 32;
-#pragma unroll
-                for (int e4 = 0; e4 < 8; ++e4) {
-                    const float4 t4 = tn4[e4];
-                    const float d0 = __fmaf_rn(-2.f, __uint_as_float(v[e4 * 4 + 0]), t4.x);
-                    const float d1 = __fmaf_rn(-2.f, __uint_as_float(v[e4 * 4 + 1]), t4.y);
-                    const float d2 = __fmaf_rn(-2.f, __uint_as_float(v[e4 * 4 + 2]), t4.z);
-                    const float d3 = __fmaf_rn(-2.f, __uint_as_float(v[e4 * 4 + 3]), t4.w);
-                    const float m = fminf(fminf(d0, d1), fminf(d2, d3));
-                    if (m < b2) {   // some lane's running second-best is displaced inside this group of four
-                        const float dd[4] = {d0, d1, d2, d3};
-#pragma unroll
-                        for (int e = 0; e < 4; ++e) {
-                            const float d = dd[e];
-                            if (d < b2) {   // usually one element of the group, in one or two lanes
-                                const int j = jc + e4 * 4 + e;
-                                const bool lt1 = d < b1;           // strict: ascending j, the lower train index wins ties
-                                i2 = lt1 ? i1 : j;
-                                b2 = lt1 ? b1 : d;
-                                i1 = lt1 ? j : i1;
-                                b1 = lt1 ? d : b1;
-                            }
-                        }
-                    }
-                }
-            }
-            tc_fence_before();
-            mbar_arrive(bar_accempty + 8 * s);
-            tau_s[rl * 4 + sub] = b2;
-            if (pre) tn_s[(s ^ 1) * KNN_BN + et] = tn_next;
-        }
-        const float qn = qnorm[row];
-        KnnPartial p;
-        p.d1 = i1 >= 0 ? __fadd_rn(b1, qn) : KNN_BIG;
-        p.d2 = i2 >= 0 ? __fadd_rn(b2, qn) : KNN_BIG;
-        p.i1 = i1; p.i2 = i2;
-        partial[((size_t)blockIdx.y * 4 + sub) * nq_pad + row] = p;
-    }
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 1) {
-        tc_fence_after();
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;" ::"r"(tmem_base) : "memory");
-    }
-}
-
-// ------------------------------------------------------------------ round 2: 256 query rows per CTA, distances inside the GEMM
-// What bounds the kernel above at 8192 x 8192 (measured with its epilogue cut short, DESIGN.md section 4): the L2 operand
-// feed -- every CTA re-streams the train descriptors, 64 KB per 128 x 256 x 128 tile -- and the scan: a compare-select
-// update path that a warp enters when ANY of its 32 rows is displaced, i.e. for about half of the four-column groups.
-// This kernel
+// ------------------------------------------------------------------ GEMM + fused top-2: 256 query rows per CTA, distances inside the GEMM
+// At 8192 x 8192 two things bound a tensor-core kNN (DESIGN.md section 4): the L2 operand feed -- every CTA streams the
+// train descriptors -- and the scan, where a compare-select update path is entered by a warp whenever ANY of its 32 rows
+// is displaced, i.e. for about half of the four-column groups.  This kernel
 //  (1) keeps TWO query tiles resident per CTA and streams train tiles of 128 rows through a 3-stage ring, so one 36 KB
-//      stage feeds two M = 128 MMAs (half the operand bytes per flop);
+//      stage feeds two M = 128 MMAs (half the operand bytes per flop of a single query tile);
 //  (2) lets the tensor core produce the finished squared distance, offset into one binade: seven extra K columns carry
 //      |t|^2 and |q|^2 as base-256 digits against {1, 256, 256} and the constant 2^23 = 4096 * 2048, so the accumulator
 //      is  d + 2^23  with d = |q|^2 + |t|^2 - 2 q.t in [0, 128 * 255^2] -- an integer in [2^23, 2^24), whose float32 bit
@@ -283,16 +76,6 @@ __device__ __forceinline__ uint64_t umma_desc_sw32(uint32_t smem_addr)
 {
     // K-major, 32-byte swizzle: rows of 32 B, 8-row groups 256 B apart
     return (uint64_t)((smem_addr >> 4) & 0x3FFF) | (1ull << 16) | (16ull << 32) | (1ull << 46) | (6ull << 61);
-}
-__device__ __forceinline__ void tc_ld_wait32(uint32_t* v)
-{
-    // wait::ld with the loaded registers as in/out operands: nothing that reads them can be scheduled above the wait
-    asm volatile("tcgen05.wait::ld.sync.aligned;"
-                 : "+r"(v[0]), "+r"(v[1]), "+r"(v[2]), "+r"(v[3]), "+r"(v[4]), "+r"(v[5]), "+r"(v[6]), "+r"(v[7]),
-                   "+r"(v[8]), "+r"(v[9]), "+r"(v[10]), "+r"(v[11]), "+r"(v[12]), "+r"(v[13]), "+r"(v[14]), "+r"(v[15]),
-                   "+r"(v[16]), "+r"(v[17]), "+r"(v[18]), "+r"(v[19]), "+r"(v[20]), "+r"(v[21]), "+r"(v[22]), "+r"(v[23]),
-                   "+r"(v[24]), "+r"(v[25]), "+r"(v[26]), "+r"(v[27]), "+r"(v[28]), "+r"(v[29]), "+r"(v[30]), "+r"(v[31])
-                 :: "memory");
 }
 __device__ __forceinline__ void tc_ld16(uint32_t taddr, uint32_t* v)
 {
@@ -362,10 +145,8 @@ knn_prep3_kernel(const float* __restrict__ src, int n, int n_pad, int is_query, 
 __global__ void __launch_bounds__(KNN_THREADS, 1)
 knn_gemm_top2_m256_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_qx,
                           const __grid_constant__ CUtensorMap map_t, const __grid_constant__ CUtensorMap map_tx,
-                          int n_tiles, int per, int total, int nt, KnnPartial* __restrict__ partial, int nq_pad, int dbg)
+                          int n_tiles, int per, int total, int nt, KnnPartial* __restrict__ partial, int nq_pad)
 {
-    // dbg (benchmarks only, B200VO_KNN_DBG): 1 = the epilogue pulls the accumulators but does not reduce them (TMEM-read
-    // floor), 2 = it hands every accumulator stage straight back (TMA + MMA floor); results are meaningless then
     extern __shared__ uint8_t smem_raw[];
     const int f0 = blockIdx.x * per, f1 = min(f0 + per, total);
     if (f0 >= f1) return;                      // uniform: before any barrier / TMEM allocation
@@ -470,14 +251,6 @@ knn_gemm_top2_m256_kernel(const __grid_constant__ CUtensorMap map_q, const __gri
         const int pad_tile = (nt % K3_BN) ? n_tiles - 1 : -1;   // the train tile that holds rows beyond nt
         int it = 0;
         uint32_t va[16], vb[16];
-        if (dbg == 2) {
-            for (int i = 0; i < f1 - f0; ++i) {
-                mbar_wait(bar_accfull + 8 * ((i & 1) * 2 + h), (i >> 1) & 1);
-                tc_fence_after();
-                tc_fence_before();
-                mbar_arrive(bar_accempty + 8 * ((i & 1) * 2 + h));
-            }
-        } else {
         {   // first 16-column piece of the first unit; from here on the pieces form one software pipeline across units and
             // segments: while a piece is reduced the next one's tcgen05.ld is in flight
             mbar_wait(bar_accfull + 8 * h, 0);
@@ -508,13 +281,6 @@ knn_gemm_top2_m256_kernel(const __grid_constant__ CUtensorMap map_q, const __gri
                     float k[16];
 #pragma unroll
                     for (int e = 0; e < 16; ++e) k[e] = __uint_as_float(v[e] * 64u + (0x80000000u | (uint32_t)(c * 16 + e)));
-                    if (dbg == 1) {
-                        uint32_t x = 0;
-#pragma unroll
-                        for (int e = 0; e < 16; ++e) x ^= v[e];
-#pragma unroll
-                        for (int e = 0; e < 16; ++e) k[e] = __uint_as_float(0x7F000000u | (x & 1u));      // keeps the loads alive, skips the network below
-                    }
                     if (c == 3 && f + (n - na) + 1 < f1) {                            // first piece of the next unit (vb's keys are built, va is free)
                         const int it2 = it + 1;
                         mbar_wait(bar_accfull + 8 * ((it2 & 1) * 2 + h), (it2 >> 1) & 1);
@@ -572,7 +338,6 @@ knn_gemm_top2_m256_kernel(const __grid_constant__ CUtensorMap map_q, const __gri
             partial[((size_t)slot * 2 + cg) * nq_pad + row] = p;
             f += nb - na;
         }
-        }   // dbg != 2
     }
     tc_fence_before();
     __syncthreads();
@@ -634,57 +399,10 @@ static int knn_make_map_ext(b200vo_ctx* ctx, CUtensorMap* map, void* gptr, int r
     return vo_encode_tiled(ctx, map, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, gptr, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_32B);
 }
 
-// the round-1 kernel (one query tile per CTA, norms added in the scan): B200VO_KNN=v1
-static int vo_knn2_ratio_dev_v1(b200vo_ctx* ctx, const float* q_dev, int nq, const float* t_dev, int nt, double ratio,
-                                int* idx2_dev, float* dist2_dev, uint8_t* accept_dev, int* bad_flag_host)
-{
-    const int nq_pad = (int)vo_align((size_t)nq, KNN_BM), nt_pad = (int)vo_align((size_t)nt, KNN_BN);
-    const int m_tiles = nq_pad / KNN_BM, n_tiles = nt_pad / KNN_BN;
-    // split the train range so that the grid covers the SMs; every split keeps tiles in ascending order
-    int n_splits = ctx->num_sms / m_tiles;   // one wave: m_tiles * n_splits <= number of SMs
-    if (n_splits > n_tiles) n_splits = n_tiles;
-    if (n_splits < 1) n_splits = 1;
-    const int tiles_per_split = (n_tiles + n_splits - 1) / n_splits;
-    n_splits = (n_tiles + tiles_per_split - 1) / tiles_per_split;
-    const size_t b_q16 = vo_align((size_t)nq_pad * KNN_DIM * 2, 1024), b_t16 = vo_align((size_t)nt_pad * KNN_DIM * 2, 1024);
-    const size_t b_qn = vo_align((size_t)nq_pad * 4, 256), b_tn = vo_align((size_t)nt_pad * 4, 256);
-    const size_t b_part = vo_align((size_t)4 * n_splits * nq_pad * sizeof(KnnPartial), 256);
-    VO_TRY(vo_reserve(ctx, ctx->d_scratch[3], b_q16 + b_t16 + b_qn + b_tn + b_part + 256));
-    uint8_t* d = (uint8_t*)ctx->d_scratch[3].p;
-    __half* q16 = (__half*)d; d += b_q16;
-    __half* t16 = (__half*)d; d += b_t16;
-    float* qn = (float*)d; d += b_qn;
-    float* tn = (float*)d; d += b_tn;
-    KnnPartial* part = (KnnPartial*)d; d += b_part;
-    int* bad = (int*)d;
-    ctx->knn_bad_flag = bad;
-    VO_CUDA(ctx, cudaMemsetAsync(bad, 0, 4, ctx->stream));
-    knn_prep_kernel<<<(nq_pad + 7) / 8, 256, 0, ctx->stream>>>(q_dev, nq, nq_pad, q16, qn, 0.f, bad);
-    knn_prep_kernel<<<(nt_pad + 7) / 8, 256, 0, ctx->stream>>>(t_dev, nt, nt_pad, t16, tn, KNN_BIG, bad);
-    ctx->launches += 2;
-    CUtensorMap map_q, map_t;
-    VO_TRY(knn_make_map(ctx, &map_q, q16, nq_pad, KNN_BM));
-    VO_TRY(knn_make_map(ctx, &map_t, t16, nt_pad, KNN_BN));
-    static bool attr_done = false;
-    if (!attr_done) {
-        VO_CUDA(ctx, cudaFuncSetAttribute(knn_gemm_top2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, KNN_SMEM));
-        attr_done = true;
-    }
-    knn_gemm_top2_kernel<<<dim3(m_tiles, n_splits), KNN_THREADS, KNN_SMEM, ctx->stream>>>(map_q, map_t, qn, tn, n_tiles, tiles_per_split,
-                                                                                       part, nq_pad);
-    knn_finalize_kernel<<<(nq + 255) / 256, 256, 0, ctx->stream>>>(part, 4 * n_splits, nq, nq_pad, nt, ratio, idx2_dev, dist2_dev, accept_dev);
-    ctx->launches += 2;
-    VO_CUDA(ctx, cudaGetLastError());
-    if (bad_flag_host) VO_CUDA(ctx, cudaMemcpyAsync(bad_flag_host, bad, 4, cudaMemcpyDeviceToHost, ctx->stream));
-    return 0;
-}
-
 // device-resident core: q_dev/t_dev float32 row-major; outputs device pointers
 int vo_knn2_ratio_dev(b200vo_ctx* ctx, const float* q_dev, int nq, const float* t_dev, int nt, double ratio,
                       int* idx2_dev, float* dist2_dev, uint8_t* accept_dev, int* bad_flag_host)
 {
-    static const bool use_v1 = getenv("B200VO_KNN") && !strcmp(getenv("B200VO_KNN"), "v1");
-    if (use_v1) return vo_knn2_ratio_dev_v1(ctx, q_dev, nq, t_dev, nt, ratio, idx2_dev, dist2_dev, accept_dev, bad_flag_host);
     const int nq_pad = (int)vo_align((size_t)nq, 2 * KNN_BM), nt_pad = (int)vo_align((size_t)nt, K3_BN);
     const int m_pairs = nq_pad / (2 * KNN_BM), n_tiles = nt_pad / K3_BN;
     // (query pair, train tile) units in query-pair-major order, one contiguous run per SM
@@ -718,9 +436,8 @@ int vo_knn2_ratio_dev(b200vo_ctx* ctx, const float* q_dev, int nq, const float* 
         VO_CUDA(ctx, cudaFuncSetAttribute(knn_gemm_top2_m256_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, K3_SMEM));
         attr_done = true;
     }
-    static const int dbg = getenv("B200VO_KNN_DBG") ? atoi(getenv("B200VO_KNN_DBG")) : 0;
     knn_gemm_top2_m256_kernel<<<(total + per - 1) / per, KNN_THREADS, K3_SMEM, ctx->stream>>>(map_q, map_qx, map_t, map_tx, n_tiles, per, total, nt,
-                                                                                               part, nq_pad, dbg);
+                                                                                               part, nq_pad);
     knn_finalize_kernel<<<(nq + 255) / 256, 256, 0, ctx->stream>>>(part, 2 * n_splits, nq, nq_pad, nt, ratio, idx2_dev, dist2_dev, accept_dev);
     ctx->launches += 2;
     VO_CUDA(ctx, cudaGetLastError());

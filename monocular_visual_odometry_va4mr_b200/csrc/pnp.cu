@@ -1010,37 +1010,35 @@ void vo_pnp_carve_workspace(PnpArgs& a, void* ws)
 
 bool vo_pnp_fused_ok(const PnpArgs& a, bool gen_samples)
 {
-    static const bool off = getenv("B200VO_POSE_UNFUSED") != nullptr;   // A/B switch for measurements
-    return !off && gen_samples && !a.full_counts && a.cap <= VO_PNP_FUSED_MAX_N;
+    return gen_samples && !a.full_counts && a.cap <= VO_PNP_FUSED_MAX_N;
 }
 
-int vo_pnp_fused_launch(b200vo_ctx* ctx, const PnpArgs& a, const PoseBatchIO& io)
+int vo_pnp_fused_launch(b200vo_ctx* ctx, const PnpArgs& a, const PoseBatchIO& io, cudaStream_t stream)
 {
     if (a.batch <= 0) return 0;
     const size_t smem = ((sizeof(PoseFusedShared) + 15) / 16) * 16 + sizeof(EpnpShared);
     static_assert(((sizeof(PoseFusedShared) + 15) / 16) * 16 + sizeof(EpnpShared) <= 48 * 1024, "static limit of dynamic shared memory");
     // few sequences: the chain's latency is the step (single sequence, small shards) -> the unconstrained build;
     // many: it runs beside the candidate tracker and must leave it registers -> two CTAs per SM
-    static const char* force = getenv("B200VO_POSE_REGS");   // "255" / "128": A/B switch for measurements
-    const bool wide = force ? atoi(force) > 128 : 2 * a.batch <= ctx->num_sms;
-    VO_CUDA(ctx, cudaMemsetAsync(a.flags, 0, (size_t)a.batch * 3 * sizeof(int), ctx->stream));
-    if (wide) pnp_fused_kernel<1><<<a.batch, FUSED_T, smem, ctx->stream>>>(a, io);
-    else pnp_fused_kernel<2><<<a.batch, FUSED_T, smem, ctx->stream>>>(a, io);
+    const bool wide = 2 * a.batch <= ctx->num_sms;
+    VO_CUDA(ctx, cudaMemsetAsync(a.flags, 0, (size_t)a.batch * 3 * sizeof(int), stream));
+    if (wide) pnp_fused_kernel<1><<<a.batch, FUSED_T, smem, stream>>>(a, io);
+    else pnp_fused_kernel<2><<<a.batch, FUSED_T, smem, stream>>>(a, io);
     ctx->launches++;
     VO_CUDA(ctx, cudaGetLastError());
     return 0;
 }
 
-int vo_pnp_launch(b200vo_ctx* ctx, const PnpArgs& a, bool gen_samples)
+int vo_pnp_launch(b200vo_ctx* ctx, const PnpArgs& a, bool gen_samples, cudaStream_t stream)
 {
     if (a.batch <= 0) return 0;
-    if (vo_pnp_fused_ok(a, gen_samples)) return vo_pnp_fused_launch(ctx, a, PoseBatchIO{});
-    VO_CUDA(ctx, cudaMemsetAsync(a.flags, 0, (size_t)a.batch * 3 * sizeof(int), ctx->stream));
+    if (vo_pnp_fused_ok(a, gen_samples)) return vo_pnp_fused_launch(ctx, a, PoseBatchIO{}, stream);
+    VO_CUDA(ctx, cudaMemsetAsync(a.flags, 0, (size_t)a.batch * 3 * sizeof(int), stream));
     if (gen_samples) {
         const size_t smem = (size_t)a.n_raw * sizeof(int);
         if (smem > 48 * 1024)
             VO_CUDA(ctx, cudaFuncSetAttribute(ransac_samples_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        ransac_samples_kernel<4><<<a.batch, 128, smem, ctx->stream>>>(a.rng_raw, a.n_raw, a.n, a.iters, a.samples, a.flags);
+        ransac_samples_kernel<4><<<a.batch, 128, smem, stream>>>(a.rng_raw, a.n_raw, a.n, a.iters, a.samples, a.flags);
         ctx->launches++;
     }
     // head chunk: the first PNP_HEAD hypotheses; its last scoring CTA per sequence leaves need[b].
@@ -1054,16 +1052,16 @@ int vo_pnp_launch(b200vo_ctx* ctx, const PnpArgs& a, bool gen_samples)
         const int nh = c.h_end - c.h_begin;
         if (nh <= 0) continue;
         dim3 g1((nh + 63) / 64, a.batch);
-        pnp_solve_kernel<<<g1, 64, 0, ctx->stream>>>(c);
+        pnp_solve_kernel<<<g1, 64, 0, stream>>>(c);
         dim3 g2((a.cap + 255) / 256, (nh + SCORE_HT - 1) / SCORE_HT, a.batch);
-        pnp_score_kernel<<<g2, 256, 0, ctx->stream>>>(c);
+        pnp_score_kernel<<<g2, 256, 0, stream>>>(c);
         ctx->launches += 2;
     }
-    pnp_select_kernel<<<a.batch, 256, 0, ctx->stream>>>(a);
+    pnp_select_kernel<<<a.batch, 256, 0, stream>>>(a);
     ctx->launches++;
     {
         const size_t smem = sizeof(EpnpShared);
-        pnp_epnp_kernel<<<a.batch, EPNP_T, smem, ctx->stream>>>(a);
+        pnp_epnp_kernel<<<a.batch, EPNP_T, smem, stream>>>(a);
         ctx->launches++;
     }
     VO_CUDA(ctx, cudaGetLastError());

@@ -1,5 +1,6 @@
 // Argument block shared by the PnP-RANSAC kernels (all pointers are device memory).
 #pragma once
+#include <cuda_runtime.h>
 #include <cstdint>
 #include <cstddef>
 
@@ -56,9 +57,9 @@ struct PoseBatchIO {
 
 void vo_rng_raw_stream(uint32_t* out, int n);
 bool vo_pnp_fused_ok(const PnpArgs& a, bool gen_samples);
-int vo_pnp_fused_launch(b200vo_ctx* ctx, const PnpArgs& a, const PoseBatchIO& io);
+int vo_pnp_fused_launch(b200vo_ctx* ctx, const PnpArgs& a, const PoseBatchIO& io, cudaStream_t stream);
 size_t vo_pnp_workspace_bytes(int batch, int cap, int iters);
 void vo_pnp_carve_workspace(PnpArgs& a, void* ws);
-int vo_pnp_launch(b200vo_ctx* ctx, const PnpArgs& a, bool gen_samples);
+int vo_pnp_launch(b200vo_ctx* ctx, const PnpArgs& a, bool gen_samples, cudaStream_t stream);
 // device table of the raw RNG stream, at least n values (grown on demand, owned by ctx)
 int vo_rng_table(b200vo_ctx* ctx, int n, const uint32_t** d_table);

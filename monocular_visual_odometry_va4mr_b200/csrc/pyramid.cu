@@ -292,14 +292,14 @@ static int pyr_src_map(b200vo_ctx* ctx, CUtensorMap* map, uint8_t* d_slab, size_
 }
 
 int vo_build_pyramids(b200vo_ctx* ctx, const uint8_t* d_raw, size_t raw_stride, int rows, int cols,
-                      const PyrGeom& g, uint8_t* d_slab, size_t slab_stride, int batch)
+                      const PyrGeom& g, uint8_t* d_slab, size_t slab_stride, int batch, cudaStream_t stream)
 {
     {
         dim3 block(32, 8);
         int gxn = (cols + 2 * VO_BORDER + 15) / 16;
         dim3 grid((gxn + block.x - 1) / block.x, (rows + 2 * VO_BORDER + block.y - 1) / block.y, batch);
-        pad_level0_kernel<<<grid, block, 0, ctx->stream>>>(d_raw, raw_stride, cols, rows, d_slab, slab_stride,
-                                                            g.off[0], g.pitch[0]);
+        pad_level0_kernel<<<grid, block, 0, stream>>>(d_raw, raw_stride, cols, rows, d_slab, slab_stride,
+                                                       g.off[0], g.pitch[0]);
         ctx->launches++;
     }
     if (g.levels > 1) {
@@ -312,14 +312,14 @@ int vo_build_pyramids(b200vo_ctx* ctx, const uint8_t* d_raw, size_t raw_stride, 
                 VO_TRY(pyr_src_map(ctx, &map, d_slab, batch == 1 ? g.slab_bytes : slab_stride, batch, g, l - 1));
                 dim3 grid((g.w[l] + PD_TW - 1) / PD_TW, (g.h[l] + PD_TH - 1) / PD_TH, batch);
                 fused = g.w[l] >= VO_BORDER + 2 && g.h[l] >= VO_BORDER + 2;   // single-bounce reflection: the tiles write the ring
-                pyr_down_tma_kernel<<<grid, 256, 0, ctx->stream>>>(map, d_slab, slab_stride, g.off[l], g.w[l], g.h[l], g.pitch[l], fused ? 1 : 0);
+                pyr_down_tma_kernel<<<grid, 256, 0, stream>>>(map, d_slab, slab_stride, g.off[l], g.w[l], g.h[l], g.pitch[l], fused ? 1 : 0);
             } else {
                 dim3 block(32, 8);
                 int gxn = (g.w[l] + 2 * VO_BORDER + 3) / 4;
                 dim3 grid((gxn + block.x - 1) / block.x, (g.h[l] + 2 * VO_BORDER + block.y - 1) / block.y, batch);
-                pyr_down_kernel<<<grid, block, 0, ctx->stream>>>(d_slab, d_slab, slab_stride, g.off[l - 1], g.w[l - 1],
-                                                                  g.h[l - 1], g.pitch[l - 1], g.off[l], g.w[l], g.h[l],
-                                                                  g.pitch[l]);
+                pyr_down_kernel<<<grid, block, 0, stream>>>(d_slab, d_slab, slab_stride, g.off[l - 1], g.w[l - 1],
+                                                             g.h[l - 1], g.pitch[l - 1], g.off[l], g.w[l], g.h[l],
+                                                             g.pitch[l]);
             }
             ctx->launches++;
             if (tma_ok && !fused) {
@@ -329,7 +329,7 @@ int vo_build_pyramids(b200vo_ctx* ctx, const uint8_t* d_raw, size_t raw_stride, 
                 for (int k = 0; k <= l; ++k) { ba.w[k] = g.w[k]; ba.h[k] = g.h[k]; ba.pitch[k] = g.pitch[k]; ba.off[k] = g.off[k]; }
                 // only level l needs filling now: launch with a single y-slice mapped onto level l
                 ba.levels = l + 1;
-                pyr_border_level_kernel<<<dim3(16, 1, batch), 256, 0, ctx->stream>>>(d_slab, slab_stride, ba, l);
+                pyr_border_level_kernel<<<dim3(16, 1, batch), 256, 0, stream>>>(d_slab, slab_stride, ba, l);
                 ctx->launches++;
             }
         }
