@@ -308,6 +308,58 @@ int b200vo_batch_good_features(b200vo_batch* b, int max_corners, double quality,
 int b200vo_batch_profile(b200vo_batch* b, int enable);
 /* Sums the recorded stage times (ms) over the *n_steps profiled steps since the last enable. */
 int b200vo_batch_profile_read(b200vo_batch* b, float* stage_ms /* [B200VO_PROF_STAGES] */, int* n_steps);
+/*
+ * ---- the whole per-frame loop on the device (INTEGRATION.md 3d) ----
+ * `continuous_operation` (:326-373) for `batch` independent sequences with the VO state of every sequence resident in
+ * device memory.  One step tracks the landmarks and the candidates into the new frame, runs P3P-RANSAC + EPnP, keeps
+ * the inliers, triangulates the candidates, detects new corners, appends the candidates that pass the distance
+ * filter and the new pose.  Only a small result block per sequence leaves the device.
+ * A sequence that cannot follow the reference's data flow stops with a status code and is skipped (its state is
+ * left as it is) until it is loaded again.
+ */
+typedef struct b200vo_loop b200vo_loop;
+typedef struct {
+    b200vo_batch_cfg batch;          /* tracker + PnP; max_landmarks / max_candidates = state capacities per sequence */
+    double min_dist_landmarks, max_dist_landmarks, min_baseline_angle_deg;   /* main.py:21-25 */
+    int min_baseline_frames;
+    int max_corners;                 /* goodFeaturesToTrack (main.py:28-33): blockSize 3, no mask, no Harris */
+    double quality_level, feature_min_dist;
+    int max_frames;                  /* pose-history capacity per sequence */
+} b200vo_loop_cfg;
+
+#define B200VO_LOOP_OK 0
+#define B200VO_LOOP_IDLE 1          /* never loaded */
+#define B200VO_LOOP_FEW_POINTS 2    /* fewer than 8 landmarks tracked (:342) */
+#define B200VO_LOOP_PNP_FAILED 3    /* solvePnPRansac found no pose (:352) */
+#define B200VO_LOOP_OVERFLOW 4      /* an append would exceed a capacity (landmarks, candidates or pose history) */
+#define B200VO_LOOP_DETECT_LIMIT 5  /* more corner candidates in the frame than the batched detector ranks */
+
+int b200vo_loop_create(b200vo_ctx* ctx, int batch, const b200vo_loop_cfg* cfg, b200vo_loop** out);
+void b200vo_loop_destroy(b200vo_loop* lp);
+/* State of sequence `seq` after its bootstrap (host arrays): frame uint8 (rows,cols) tight = the current frame;
+ * lm float32 (n_lm,3) + lm_kp float32 (n_lm,2); keys / first_keys float32 (n_cand,2) + first_pose int32 (n_cand)
+ * = potential_keys / potential_first_keys / potential_transforms; poses double (n_poses,12) = self.transforms as
+ * (R_CW row-major | t_CW).  The sequence's status becomes B200VO_LOOP_OK.  Synchronous. */
+int b200vo_loop_load(b200vo_loop* lp, int seq, const uint8_t* frame, const float* lm, const float* lm_kp, int n_lm,
+                     const float* keys, const float* first_keys, const int32_t* first_pose, int n_cand,
+                     const double* poses, int n_poses);
+/* The same arrays back (capacity-sized outputs: max_landmarks, max_candidates, max_frames rows), plus the counts and
+ * the status.  Synchronous. */
+int b200vo_loop_read_state(b200vo_loop* lp, int seq, float* lm, float* lm_kp, int32_t* n_lm, float* keys, float* first_keys,
+                           int32_t* first_pose, int32_t* n_cand, double* poses, int32_t* n_poses, int32_t* status);
+/* Frames of a future step, as b200vo_batch_submit_frames(_dev). */
+int b200vo_loop_submit_frames(b200vo_loop* lp, const uint8_t* frames);
+int b200vo_loop_submit_frames_dev(b200vo_loop* lp, const uint8_t* frames_dev);
+/* One frame for every sequence (frames: batch x rows x cols uint8; NULL: the oldest submitted set).
+ * Per sequence: status int32, n_inliers int32, n_lm int32, n_cand int32 after the step, pose_cw double (batch,12) =
+ * the pose appended this step.  n_inliers and pose_cw are 0 unless status is B200VO_LOOP_OK.
+ * One upload (the frames, unless submitted) and one read-back of the packed result block. */
+int b200vo_loop_step(b200vo_loop* lp, const uint8_t* frames, int32_t* status, int32_t* n_inliers, int32_t* n_lm,
+                     int32_t* n_cand, double* pose_cw);
+/* The same with device pointers; asynchronous on the ctx stream (never synchronises the host). */
+int b200vo_loop_step_dev(b200vo_loop* lp, const uint8_t* frames_dev, int32_t* status_dev, int32_t* n_inliers_dev,
+                         int32_t* n_lm_dev, int32_t* n_cand_dev, double* pose_cw_dev);
+
 int b200vo_sync(b200vo_ctx* ctx);
 /* Page-locked host memory for frame buffers: b200vo_batch_step DMAs straight out of such a
  * buffer (pageable memory is staged through an internal pinned copy first). */

@@ -32,6 +32,16 @@ class BatchCfg(C.Structure):
     ]
 
 
+class LoopCfg(C.Structure):
+    _fields_ = [
+        ("batch", BatchCfg),
+        ("min_dist_landmarks", C.c_double), ("max_dist_landmarks", C.c_double), ("min_baseline_angle_deg", C.c_double),
+        ("min_baseline_frames", C.c_int),
+        ("max_corners", C.c_int), ("quality_level", C.c_double), ("feature_min_dist", C.c_double),
+        ("max_frames", C.c_int),
+    ]
+
+
 # name -> (restype, argtypes); mirrors include/b200vo.h one to one
 SIGNATURES = {
     "b200vo_create": (C.c_int, [C.c_int, C.POINTER(C.c_void_p)]),
@@ -103,6 +113,16 @@ SIGNATURES = {
     "b200vo_batch_step_dev": (C.c_int, [C.c_void_p] + [C.c_void_p] * 14),
     "b200vo_batch_profile": (C.c_int, [C.c_void_p, C.c_int]),
     "b200vo_batch_profile_read": (C.c_int, [C.c_void_p, c_f32p, c_intp]),
+    "b200vo_loop_create": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(LoopCfg), C.POINTER(C.c_void_p)]),
+    "b200vo_loop_destroy": (None, [C.c_void_p]),
+    "b200vo_loop_load": (C.c_int, [C.c_void_p, C.c_int, c_u8p, c_f32p, c_f32p, C.c_int, c_f32p, c_f32p, c_i32p, C.c_int, c_f64p,
+                                   C.c_int]),
+    "b200vo_loop_read_state": (C.c_int, [C.c_void_p, C.c_int, c_f32p, c_f32p, c_i32p, c_f32p, c_f32p, c_i32p, c_i32p, c_f64p, c_i32p,
+                                         c_i32p]),
+    "b200vo_loop_submit_frames": (C.c_int, [C.c_void_p, c_u8p]),
+    "b200vo_loop_submit_frames_dev": (C.c_int, [C.c_void_p, C.c_void_p]),
+    "b200vo_loop_step": (C.c_int, [C.c_void_p, c_u8p, c_i32p, c_i32p, c_i32p, c_i32p, c_f64p]),
+    "b200vo_loop_step_dev": (C.c_int, [C.c_void_p] + [C.c_void_p] * 6),
     "b200vo_sync": (C.c_int, [C.c_void_p]),
     "b200vo_host_alloc": (C.c_void_p, [C.c_void_p, C.c_size_t]),
     "b200vo_host_free": (None, [C.c_void_p, C.c_void_p]),

@@ -178,3 +178,182 @@ class SequenceBatch:
             o["lm_next"], o["lm_status"], o["cand_next"], o["cand_status"], o["pose"], o["pnp_ok"],
             o["inlier_mask"], o["n_inliers"])
         self._chk(rc, "b200vo_batch_step_dev")
+
+
+def _loop_cfg(rows, cols, K, options, max_landmarks, max_candidates, max_frames):
+    o = options
+    cfg = _lib.LoopCfg()
+    bc = cfg.batch
+    bc.rows, bc.cols = int(rows), int(cols)
+    bc.win_w, bc.win_h, bc.max_level = int(o['winSize'][0]), int(o['winSize'][1]), int(o['maxLevel'])
+    bc.crit_type, bc.crit_max_count, bc.crit_eps = int(o['criteria'][0]), int(o['criteria'][1]), float(o['criteria'][2])
+    bc.min_eig_thr = 1e-4                          # cv2.calcOpticalFlowPyrLK's default (the reference passes none)
+    bc.pnp_iters, bc.pnp_reproj_err, bc.pnp_conf = int(o['PnP_iterations']), float(o['PnP_error']), float(o['PnP_conf'])
+    Kf = np.asarray(K, np.float64).reshape(9)
+    for i in range(9):
+        bc.K[i] = float(Kf[i])
+    bc.max_landmarks, bc.max_candidates = int(max_landmarks), int(max_candidates)
+    cfg.min_dist_landmarks, cfg.max_dist_landmarks = float(o['min_dist_landmarks']), float(o['max_dist_landmarks'])
+    cfg.min_baseline_angle_deg, cfg.min_baseline_frames = float(o['min_baseline_angle']), int(o['min_baseline_frames'])
+    if o.get('feature_block_size', 3) != 3 or o.get('feature_use_harris', False):
+        raise NotImplementedError("VOBatch detects corners with blockSize 3 and no Harris detector (the reference's options)")
+    cfg.max_corners, cfg.quality_level = int(o['feature_max_corners']), float(o['feature_quality_level'])
+    cfg.feature_min_dist = float(o['feature_min_dist'])
+    cfg.max_frames = int(max_frames)
+    return cfg
+
+
+class VOBatch:
+    """The whole per-frame loop of the reference (``continuous_operation``, ``VisualOdometryPipeLine.py:326-373``) for
+    ``batch`` independent sequences, with the VO state of every sequence resident on the device (``b200vo_loop_*``).
+
+    ``options`` is the reference's option dict (main.py:20-44).  Each sequence is loaded once with the state its
+    bootstrap produced (``initial_state``) and then advanced one frame per ``step``.  The state of a sequence is
+    ``lm`` float32 (n_lm,3), ``lm_kp`` float32 (n_lm,2), the candidates ``keys`` / ``first_keys`` float32 (n_cand,2)
+    and ``first_pose`` int32 (n_cand,), and ``poses`` float64 (n_poses,12) = ``self.transforms`` as (R_CW | t_CW).
+    A sequence that cannot follow the reference's data flow stops with one of the status codes below and stays as it
+    is until it is loaded again."""
+
+    OK, IDLE, FEW_POINTS, PNP_FAILED, OVERFLOW, DETECT_LIMIT = range(6)
+
+    def __init__(self, batch, rows, cols, K, options, max_landmarks=4096, max_candidates=8192, max_frames=1024,
+                 ctx: _lib.Context | None = None):
+        self.ctx = ctx or _lib.default_context(0)
+        self.batch, self.rows, self.cols = int(batch), int(rows), int(cols)
+        self.L, self.Cn, self.P = int(max_landmarks), int(max_candidates), int(max_frames)
+        self.cfg = _loop_cfg(rows, cols, K, options, max_landmarks, max_candidates, max_frames)
+        h = C.c_void_p()
+        rc = self.ctx.lib.b200vo_loop_create(self.ctx.h, self.batch, C.byref(self.cfg), C.byref(h))
+        if rc != 0:
+            raise _lib.B200VOError(f"b200vo_loop_create failed ({rc}): {self.ctx.last_error()}")
+        self.h = h
+        b = self.batch
+        self._res = dict(status=self.pinned_empty((b,), np.int32), n_inliers=self.pinned_empty((b,), np.int32),
+                         n_lm=self.pinned_empty((b,), np.int32), n_cand=self.pinned_empty((b,), np.int32),
+                         pose_cw=self.pinned_empty((b, 12), np.float64))
+        r = self._res
+        self._res_ptrs = (_p(r['status'], c_i32p), _p(r['n_inliers'], c_i32p), _p(r['n_lm'], c_i32p), _p(r['n_cand'], c_i32p),
+                          _p(r['pose_cw'], c_f64p))
+
+    def close(self):
+        if getattr(self, "h", None):
+            self.ctx.lib.b200vo_loop_destroy(self.h)
+            self.h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def _chk(self, rc, what):
+        if rc == -1:
+            raise ValueError(f"{what}: {self.ctx.last_error()}")
+        if rc != 0:
+            raise _lib.B200VOError(f"{what} failed ({rc}): {self.ctx.last_error()}")
+
+    def pinned_empty(self, shape, dtype) -> np.ndarray:
+        """numpy array in page-locked host memory (b200vo_host_alloc)."""
+        dt = np.dtype(dtype)
+        return _PinnedBlock(self.ctx, max(int(np.prod(shape)) * dt.itemsize, 1)).array(shape, dt)
+
+    def pinned_frames(self, n_sets: int = 1) -> np.ndarray:
+        """(n_sets, batch, rows, cols) uint8 array in page-locked memory, for submit_frames() and step()."""
+        return self.pinned_empty((n_sets, self.batch, self.rows, self.cols), np.uint8)
+
+    def load(self, seq: int, frame: np.ndarray, state: dict):
+        """Set sequence ``seq`` to ``state`` (see the class docstring) with ``frame`` as its current frame; its status
+        becomes OK.  Out-of-range counts or first_pose values raise ValueError and change nothing."""
+        f = np.ascontiguousarray(frame, np.uint8)
+        if f.shape != (self.rows, self.cols):
+            raise ValueError(f"frame must be ({self.rows}, {self.cols}) uint8")
+        lm = np.ascontiguousarray(state['lm'], np.float32).reshape(-1, 3)
+        kp = np.ascontiguousarray(state['lm_kp'], np.float32).reshape(-1, 2)
+        keys = np.ascontiguousarray(state['keys'], np.float32).reshape(-1, 2)
+        fk = np.ascontiguousarray(state['first_keys'], np.float32).reshape(-1, 2)
+        fp = np.ascontiguousarray(state['first_pose'], np.int32).reshape(-1)
+        poses = np.ascontiguousarray(state['poses'], np.float64).reshape(-1, 12)
+        if len(kp) != len(lm) or len(fk) != len(keys) or len(fp) != len(keys):
+            raise ValueError("lm / lm_kp and keys / first_keys / first_pose must have one row per point")
+        self._chk(self.ctx.lib.b200vo_loop_load(self.h, int(seq), _p(f, c_u8p), _p(lm, c_f32p), _p(kp, c_f32p), len(lm),
+                                                _p(keys, c_f32p), _p(fk, c_f32p), _p(fp, c_i32p), len(keys), _p(poses, c_f64p),
+                                                len(poses)), "b200vo_loop_load")
+
+    def read_state(self, seq: int) -> dict:
+        """The state of sequence ``seq`` (copies) and its ``status``."""
+        lm = np.zeros((self.L, 3), np.float32)
+        kp = np.zeros((self.L, 2), np.float32)
+        keys = np.zeros((self.Cn, 2), np.float32)
+        fk = np.zeros((self.Cn, 2), np.float32)
+        fp = np.zeros(self.Cn, np.int32)
+        poses = np.zeros((self.P, 12), np.float64)
+        n_lm, n_cand, n_poses, status = (C.c_int32(0) for _ in range(4))
+        self._chk(self.ctx.lib.b200vo_loop_read_state(self.h, int(seq), _p(lm, c_f32p), _p(kp, c_f32p), C.byref(n_lm), _p(keys, c_f32p),
+                                                      _p(fk, c_f32p), _p(fp, c_i32p), C.byref(n_cand), _p(poses, c_f64p),
+                                                      C.byref(n_poses), C.byref(status)), "b200vo_loop_read_state")
+        nl, nc, npo = n_lm.value, n_cand.value, n_poses.value
+        return dict(lm=lm[:nl], lm_kp=kp[:nl], keys=keys[:nc], first_keys=fk[:nc], first_pose=fp[:nc], poses=poses[:npo],
+                    status=status.value)
+
+    def submit_frames(self, frames: np.ndarray):
+        """Frames of a FUTURE step (page-locked, from pinned_frames()); step(None) consumes them, oldest first."""
+        assert frames.dtype == np.uint8 and frames.flags.c_contiguous and frames.size == self.batch * self.rows * self.cols
+        self._chk(self.ctx.lib.b200vo_loop_submit_frames(self.h, _p(frames, c_u8p)), "b200vo_loop_submit_frames")
+
+    def submit_frames_dev(self, frames_dev: int):
+        """The same for frames resident in device memory (int from tensor.data_ptr()); step_dev(None, ...) consumes them."""
+        self._chk(self.ctx.lib.b200vo_loop_submit_frames_dev(self.h, frames_dev), "b200vo_loop_submit_frames_dev")
+
+    def step(self, frames=None) -> dict:
+        """One frame for every sequence (frames (batch, rows, cols) uint8; None: the oldest submitted set).  Synchronous.
+        Returns views on REUSED page-locked arrays: status, n_inliers, n_lm, n_cand int32 (batch,) and pose_cw float64
+        (batch, 12), the pose appended this step (0 unless status is OK)."""
+        if frames is not None:
+            frames = np.ascontiguousarray(frames, np.uint8)
+            assert frames.size == self.batch * self.rows * self.cols
+        self._chk(self.ctx.lib.b200vo_loop_step(self.h, _p(frames, c_u8p) if frames is not None else None, *self._res_ptrs),
+                  "b200vo_loop_step")
+        return self._res
+
+    def step_dev(self, frames_dev, out_dev: dict):
+        """Device pointers (ints from tensor.data_ptr()) for the frames (None: the oldest submitted set) and for the results
+        ``status``, ``n_inliers``, ``n_lm``, ``n_cand`` (int32 (batch,)) and ``pose_cw`` (float64 (batch, 12)).
+        Asynchronous on the ctx stream."""
+        o = out_dev
+        self._chk(self.ctx.lib.b200vo_loop_step_dev(self.h, frames_dev or None, o['status'], o['n_inliers'], o['n_lm'], o['n_cand'],
+                                                    o['pose_cw']), "b200vo_loop_step_dev")
+
+
+def match_bootstrap_frames(frame0, frame1, ratio=0.8):
+    """The reference's bootstrap matching (``VisualOdometryPipeLine.py:209-245``) on the CUDA path: SIFT
+    detectAndCompute on both frames, knnMatch(k=2) and the ratio test.  -> (pts0, pts1) float32 (n, 2)."""
+    from . import cv2_compat
+    sift = cv2_compat.SIFT_create()
+    kp0, d0 = sift.detectAndCompute(frame0, None)
+    kp1, d1 = sift.detectAndCompute(frame1, None)
+    good = [m for m, n in cv2_compat.BFMatcher().knnMatch(d0, d1, k=2) if m.distance < ratio * n.distance]
+    pts0 = np.float32([kp0[m.queryIdx].pt for m in good]).reshape(-1, 2)
+    pts1 = np.float32([kp1[m.trainIdx].pt for m in good]).reshape(-1, 2)
+    return pts0, pts1
+
+
+def initial_state(K, options, first_keys, keys) -> dict:
+    """The state ``initialization`` (:295-330) leaves behind, from the bootstrap matches: findEssentialMat -> inlier split
+    -> recoverPose -> t * sign(t_z) (:317) -> triangulation of the inliers against the first pose (I, 0).
+    -> a state dict for ``VOBatch.load`` (two poses), plus ``num_pts`` = the essential-matrix inlier count."""
+    from . import cv2_compat, hotpath
+    K = np.asarray(K, np.float64).reshape(3, 3)
+    first_keys = np.ascontiguousarray(first_keys, np.float32).reshape(-1, 2)
+    keys = np.ascontiguousarray(keys, np.float32).reshape(-1, 2)
+    E, mask = cv2_compat.findEssentialMat(first_keys, keys, K, method=cv2_compat.RANSAC, prob=0.99, threshold=1.0)
+    if E is None:
+        raise ValueError("findEssentialMat found no essential matrix in the bootstrap matches")
+    inl = mask.ravel() == 1
+    pf, pk = first_keys[inl], keys[inl]
+    pt = np.zeros(len(pk), np.int32)
+    _, R, t, _ = cv2_compat.recoverPose(E, pf, pk, K)
+    t = t * np.sign(t[2])
+    poses = hotpath.pack_poses([(np.eye(3), np.zeros((3, 1))), (R, t)])
+    too_short, lm, lm_kp = hotpath.triangulate_landmarks(K, options, pf, pk, pt, poses[:1], R, t)
+    return dict(lm=lm, lm_kp=lm_kp, keys=pk[too_short], first_keys=pf[too_short], first_pose=pt[too_short], poses=poses,
+                num_pts=int(inl.sum()))

@@ -9,7 +9,7 @@
 //       (:149-168); accepted landmarks and their keypoints appended in candidate order.
 // The reference spends ~67 ms (f1) and ~48 ms (f2) per frame on these in Python loops
 // (SURVEY.md 8f); here each is one or two small launches.
-#include "internal.cuh"
+#include "landmarks.cuh"
 #include "mathdev.cuh"
 
 using namespace vo;
@@ -35,19 +35,6 @@ min_distance_kernel(const float2* __restrict__ pts, int n, const float2* __restr
     }
     if (lane == 0) valid[i] = ok ? 1 : 0;
 }
-
-struct TriArgs {
-    double K[9], Ki[9];
-    double cur[12];            // R_CW | t_CW of the current frame (as the reference stores them)
-    double min_dist, max_dist, min_angle_deg;
-    int min_frames, n, n_poses;
-    const float* first_keys; const float* keys; const int* first_pose;
-    const double* poses;       // [n_poses][12]
-    uint8_t* keep;             // [n] too_short_baseline
-    float* lm_slot;            // [n][3] per-candidate result
-    float* out_lm; float* out_kp; int* n_new;   // compacted
-    int* flags;                // bit0: first_pose out of range
-};
 
 __device__ __forceinline__ void invert_pose(const double* cw, double* R, double* t)
 {
@@ -164,17 +151,6 @@ triangulate_compact_kernel(TriArgs a) { triangulate_compact_block(a); }
 
 // ---- batched forms (SURVEY 8f "batched f1/f2 on the resident batch state"): the same per-sequence work for every
 // sequence of a batch in one launch each; blockIdx.y = sequence, ragged counts per sequence ----
-struct TriBatchArgs {
-    TriArgs common;            // K, Ki, gates (the per-sequence fields are filled in by the kernels)
-    int cap, pose_cap;
-    const int* n;              // [batch] candidates per sequence
-    const int* n_poses;        // [batch]
-    const double* cur;         // [batch][12]
-    const float* first_keys; const float* keys; const int* first_pose;   // [batch][cap]...
-    const double* poses;       // [batch][pose_cap][12]
-    uint8_t* keep; float* lm_slot; float* out_lm; float* out_kp; int* n_new; int* flags;   // [batch]...
-};
-
 __device__ __forceinline__ TriArgs tri_sequence(const TriBatchArgs& b, int s)
 {
     TriArgs a = b.common;
@@ -227,6 +203,34 @@ min_distance_batch_kernel(const float2* __restrict__ pts, const int* __restrict_
         if (!__all_sync(0xffffffffu, ok)) { ok = false; break; }
     }
     if (lane == 0) valid[(size_t)s * n_cap + i] = ok ? 1 : 0;
+}
+
+void vo_tri_common(TriArgs& c, const double K[9], double min_dist, double max_dist, double min_angle_deg, int min_frames)
+{
+    for (int k = 0; k < 9; ++k) c.K[k] = K[k];
+    const double Ki[9] = {1.0 / K[0], 0, -K[2] / K[0], 0, 1.0 / K[4], -K[5] / K[4], 0, 0, 1};
+    for (int k = 0; k < 9; ++k) c.Ki[k] = Ki[k];
+    c.min_dist = min_dist; c.max_dist = max_dist; c.min_angle_deg = min_angle_deg;
+    c.min_frames = min_frames;
+}
+
+int vo_triangulate_batch_launch(b200vo_ctx* ctx, const TriBatchArgs& b, int batch, cudaStream_t stream)
+{
+    triangulate_batch_kernel<<<dim3((b.cap + 63) / 64, batch), 64, 0, stream>>>(b);
+    triangulate_compact_batch_kernel<<<batch, 1024, 0, stream>>>(b);
+    ctx->launches += 2;
+    VO_CUDA(ctx, cudaGetLastError());
+    return 0;
+}
+
+int vo_min_distance_batch_launch(b200vo_ctx* ctx, int batch, const float* pts, const int* n, int n_cap, const float* existing,
+                                 const int* m, int m_cap, float min_dist, uint8_t* valid, cudaStream_t stream)
+{
+    min_distance_batch_kernel<<<dim3((n_cap * 32 + 255) / 256, batch), 256, 0, stream>>>(
+        (const float2*)pts, n, n_cap, (const float2*)existing, m, m_cap, min_dist, valid);
+    ctx->launches++;
+    VO_CUDA(ctx, cudaGetLastError());
+    return 0;
 }
 
 extern "C" int b200vo_min_distance_mask(b200vo_ctx* ctx, const float* pts, int n, const float* existing, int m,
@@ -338,10 +342,8 @@ extern "C" int b200vo_batch_min_distance_mask(b200vo_ctx* ctx, int batch, const 
     VO_CUDA(ctx, cudaMemcpyAsync(d, hp, b_p + b_e + 2 * b_c, cudaMemcpyHostToDevice, ctx->stream));
     uint8_t* dv = d + b_p + b_e + 2 * b_c;
     VO_CUDA(ctx, cudaMemsetAsync(dv, 0, b_v, ctx->stream));
-    min_distance_batch_kernel<<<dim3((n_cap * 32 + 255) / 256, batch), 256, 0, ctx->stream>>>(
-        (const float2*)d, (const int*)(d + b_p + b_e), n_cap, (const float2*)(d + b_p), (const int*)(d + b_p + b_e + b_c), m_cap, min_dist, dv);
-    ctx->launches++;
-    VO_CUDA(ctx, cudaGetLastError());
+    VO_TRY(vo_min_distance_batch_launch(ctx, batch, (const float*)d, (const int*)(d + b_p + b_e), n_cap, (const float*)(d + b_p),
+                                        (const int*)(d + b_p + b_e + b_c), m_cap, min_dist, dv, ctx->stream));
     uint8_t* ho = hp + b_p + b_e + 2 * b_c;
     VO_CUDA(ctx, cudaMemcpyAsync(ho, dv, (size_t)batch * n_cap, cudaMemcpyDeviceToHost, ctx->stream));
     VO_CUDA(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
@@ -368,11 +370,7 @@ extern "C" int b200vo_batch_triangulate_landmarks(b200vo_ctx* ctx, const double 
     VO_CUDA(ctx, cudaSetDevice(ctx->device));
     VO_CUDA(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
     TriBatchArgs b{};
-    for (int k = 0; k < 9; ++k) b.common.K[k] = K[k];
-    const double Ki[9] = {1.0 / K[0], 0, -K[2] / K[0], 0, 1.0 / K[4], -K[5] / K[4], 0, 0, 1};
-    for (int k = 0; k < 9; ++k) b.common.Ki[k] = Ki[k];
-    b.common.min_dist = min_dist; b.common.max_dist = max_dist; b.common.min_angle_deg = min_baseline_angle_deg;
-    b.common.min_frames = min_baseline_frames;
+    vo_tri_common(b.common, K, min_dist, max_dist, min_baseline_angle_deg, min_baseline_frames);
     b.cap = cap; b.pose_cap = pose_cap;
     const size_t nc = (size_t)batch * cap;
     const size_t b_k = vo_align(nc * 8, 256), b_fp = vo_align(nc * 4, 256), b_ps = vo_align((size_t)batch * pose_cap * 96, 256);
@@ -397,10 +395,7 @@ extern "C" int b200vo_batch_triangulate_landmarks(b200vo_ctx* ctx, const double 
     b.n_new = (int*)(dout + b_keep + b_lm + b_k); b.flags = (int*)(dout + b_keep + b_lm + b_k + b_cnt);
     b.lm_slot = (float*)(dout + out_bytes);
     VO_CUDA(ctx, cudaMemsetAsync(dout, 0, out_bytes, ctx->stream));
-    triangulate_batch_kernel<<<dim3((cap + 63) / 64, batch), 64, 0, ctx->stream>>>(b);
-    triangulate_compact_batch_kernel<<<batch, 1024, 0, ctx->stream>>>(b);
-    ctx->launches += 2;
-    VO_CUDA(ctx, cudaGetLastError());
+    VO_TRY(vo_triangulate_batch_launch(ctx, b, batch, ctx->stream));
     uint8_t* ho = hp + in_bytes;
     VO_CUDA(ctx, cudaMemcpyAsync(ho, dout, out_bytes, cudaMemcpyDeviceToHost, ctx->stream));
     VO_CUDA(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
