@@ -333,6 +333,7 @@ typedef struct {
 #define B200VO_LOOP_PNP_FAILED 3    /* solvePnPRansac found no pose (:352) */
 #define B200VO_LOOP_OVERFLOW 4      /* an append would exceed a capacity (landmarks, candidates or pose history) */
 #define B200VO_LOOP_DETECT_LIMIT 5  /* more corner candidates in the frame than the batched detector ranks */
+#define B200VO_LOOP_NO_BOOTSTRAP 6  /* the bootstrap found no essential matrix (fewer than 5 ratio-test matches, or RANSAC found no model) */
 
 int b200vo_loop_create(b200vo_ctx* ctx, int batch, const b200vo_loop_cfg* cfg, b200vo_loop** out);
 void b200vo_loop_destroy(b200vo_loop* lp);
@@ -343,6 +344,21 @@ void b200vo_loop_destroy(b200vo_loop* lp);
 int b200vo_loop_load(b200vo_loop* lp, int seq, const uint8_t* frame, const float* lm, const float* lm_kp, int n_lm,
                      const float* keys, const float* first_keys, const int32_t* first_pose, int n_cand,
                      const double* poses, int n_poses);
+/* The reference's bootstrap (`initialization`, :209-245 and :295-330) for the n_seq distinct sequences seqs[], on the device:
+ * SIFT on both frames, kNN(k=2) + ratio test (m.distance < ratio * n.distance), findEssentialMat(RANSAC, prob 0.99,
+ * threshold 1.0, maxIters 1000), recoverPose (distanceThresh 50) on the inliers, t * sign(t_z), triangulation of the inliers
+ * against [I | 0].  frames0 / frames1: uint8 [n_seq][rows][cols] host arrays (page-locked or pageable); frames1[k] becomes
+ * sequence seqs[k]'s current frame.  On success the sequence holds exactly what b200vo_loop_load would give it from that
+ * result (two poses) and its status is B200VO_LOOP_OK.  Per listed sequence: status (OK, NO_BOOTSTRAP or OVERFLOW: the
+ * landmarks exceed max_landmarks or the too_short_baseline candidates max_candidates), num_pts = the essential-matrix
+ * inlier count (0 for NO_BOOTSTRAP), n_lm / n_cand = the loaded counts (0 unless OK).  A sequence that fails keeps its
+ * state arrays, takes the status and is skipped by steps until it is loaded or bootstrapped again.  Sequences not listed
+ * are untouched.  Bad indices (out of range, repeated), n_seq < 1 or null arrays: B200VO_E_BADARG before any device work.
+ * A sequence whose RANSAC subset draw exhausts the fixed table of cv2 random numbers also gets NO_BOOTSTRAP.
+ * Synchronous; synchronises the host twice per SIFT chunk of frames plus three times, and once more per workspace that
+ * has to grow. */
+int b200vo_loop_bootstrap(b200vo_loop* lp, int n_seq, const int32_t* seqs, const uint8_t* frames0, const uint8_t* frames1,
+                          double ratio, int32_t* status, int32_t* num_pts, int32_t* n_lm, int32_t* n_cand);
 /* The same arrays back (capacity-sized outputs: max_landmarks, max_candidates, max_frames rows), plus the counts and
  * the status.  Synchronous. */
 int b200vo_loop_read_state(b200vo_loop* lp, int seq, float* lm, float* lm_kp, int32_t* n_lm, float* keys, float* first_keys,

@@ -119,6 +119,7 @@ SIGNATURES = {
                                    C.c_int]),
     "b200vo_loop_read_state": (C.c_int, [C.c_void_p, C.c_int, c_f32p, c_f32p, c_i32p, c_f32p, c_f32p, c_i32p, c_i32p, c_f64p, c_i32p,
                                          c_i32p]),
+    "b200vo_loop_bootstrap": (C.c_int, [C.c_void_p, C.c_int, c_i32p, c_u8p, c_u8p, C.c_double, c_i32p, c_i32p, c_i32p, c_i32p]),
     "b200vo_loop_submit_frames": (C.c_int, [C.c_void_p, c_u8p]),
     "b200vo_loop_submit_frames_dev": (C.c_int, [C.c_void_p, C.c_void_p]),
     "b200vo_loop_step": (C.c_int, [C.c_void_p, c_u8p, c_i32p, c_i32p, c_i32p, c_i32p, c_f64p]),

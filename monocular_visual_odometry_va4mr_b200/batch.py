@@ -212,15 +212,17 @@ class VOBatch:
     ``lm`` float32 (n_lm,3), ``lm_kp`` float32 (n_lm,2), the candidates ``keys`` / ``first_keys`` float32 (n_cand,2)
     and ``first_pose`` int32 (n_cand,), and ``poses`` float64 (n_poses,12) = ``self.transforms`` as (R_CW | t_CW).
     A sequence that cannot follow the reference's data flow stops with one of the status codes below and stays as it
-    is until it is loaded again."""
+    is until it is loaded again.  ``bootstrap`` runs the reference's bootstrap for any subset of the sequences on the
+    device instead of ``load``; a sequence whose bootstrap finds no essential matrix gets ``NO_BOOTSTRAP``."""
 
-    OK, IDLE, FEW_POINTS, PNP_FAILED, OVERFLOW, DETECT_LIMIT = range(6)
+    OK, IDLE, FEW_POINTS, PNP_FAILED, OVERFLOW, DETECT_LIMIT, NO_BOOTSTRAP = range(7)
 
     def __init__(self, batch, rows, cols, K, options, max_landmarks=4096, max_candidates=8192, max_frames=1024,
                  ctx: _lib.Context | None = None):
         self.ctx = ctx or _lib.default_context(0)
         self.batch, self.rows, self.cols = int(batch), int(rows), int(cols)
         self.L, self.Cn, self.P = int(max_landmarks), int(max_candidates), int(max_frames)
+        self.options = options
         self.cfg = _loop_cfg(rows, cols, K, options, max_landmarks, max_candidates, max_frames)
         h = C.c_void_p()
         rc = self.ctx.lib.b200vo_loop_create(self.ctx.h, self.batch, C.byref(self.cfg), C.byref(h))
@@ -278,6 +280,27 @@ class VOBatch:
         self._chk(self.ctx.lib.b200vo_loop_load(self.h, int(seq), _p(f, c_u8p), _p(lm, c_f32p), _p(kp, c_f32p), len(lm),
                                                 _p(keys, c_f32p), _p(fk, c_f32p), _p(fp, c_i32p), len(keys), _p(poses, c_f64p),
                                                 len(poses)), "b200vo_loop_load")
+
+    def bootstrap(self, frames0, frames1, seqs=None) -> dict:
+        """The reference's bootstrap (``initialization``) on the device for the sequences ``seqs`` (distinct indices; None:
+        every sequence) from their two bootstrap frames ``frames0`` / ``frames1`` (len(seqs), rows, cols) uint8, with the
+        ratio ``options['feature_ratio']``.  A sequence that succeeds ends up exactly as ``load(s, frames1[k],
+        initial_state(K, options, *match_bootstrap_frames(frames0[k], frames1[k], ratio)))`` leaves it.  Returns int32
+        arrays (len(seqs),): ``status`` (OK, NO_BOOTSTRAP or OVERFLOW), ``num_pts`` (the essential-matrix inlier count),
+        ``n_lm`` and ``n_cand``.  A failing sequence keeps its state and is skipped by ``step`` until it is loaded or
+        bootstrapped again.  Bad indices or frame shapes raise ValueError and change nothing.  Synchronous."""
+        seqs = np.arange(self.batch, dtype=np.int32) if seqs is None else np.ascontiguousarray(seqs, np.int32).reshape(-1)
+        f0 = np.ascontiguousarray(frames0, np.uint8)
+        f1 = np.ascontiguousarray(frames1, np.uint8)
+        shape = (len(seqs), self.rows, self.cols)
+        if f0.shape != shape or f1.shape != shape:
+            raise ValueError(f"frames0 and frames1 must be {shape} uint8")
+        n = len(seqs)
+        out = {k: np.zeros(max(n, 1), np.int32) for k in ('status', 'num_pts', 'n_lm', 'n_cand')}
+        self._chk(self.ctx.lib.b200vo_loop_bootstrap(self.h, n, _p(seqs, c_i32p), _p(f0, c_u8p), _p(f1, c_u8p),
+                                                     float(self.options['feature_ratio']), *(_p(out[k], c_i32p) for k in out)),
+                  "b200vo_loop_bootstrap")
+        return {k: v[:n] for k, v in out.items()}
 
     def read_state(self, seq: int) -> dict:
         """The state of sequence ``seq`` (copies) and its ``status``."""

@@ -91,6 +91,7 @@ extern "C" void b200vo_destroy(b200vo_ctx* ctx)
     for (auto& s : ctx->slots) if (s.slab.p) cudaFree(s.slab.p);
     if (ctx->d_rng.p) cudaFree(ctx->d_rng.p);
     if (ctx->d_sift.p) cudaFree(ctx->d_sift.p);
+    for (DevBuf* b : {&ctx->d_sift_out[0], &ctx->d_sift_out[1], &ctx->d_sift_sort}) if (b->p) cudaFree(b->p);
     if (ctx->d_klt_queue.p) cudaFree(ctx->d_klt_queue.p);
     if (ctx->h_pin) cudaFreeHost(ctx->h_pin);
     cudaEventDestroy(ctx->ev0);

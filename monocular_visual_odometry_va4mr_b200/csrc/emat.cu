@@ -15,7 +15,9 @@
 //                           adaptive iteration bound; hypotheses go through in chunks of 64, 128, 256, ... and a
 //                           chunk beyond the bound exits at once (cv2 stops after 10-60 samples)
 //   emat_finish_kernel      the winner's E and mask
-#include "internal.cuh"
+// Every kernel runs for a batch of independent point sets (sequences) at once, the sequence taken from the grid; each one
+// replays cv2's RNG stream and adaptive stop on its own.  One call is the batch of one.
+#include "emat.cuh"
 #include "mathdev.cuh"
 #include "ransac.cuh"
 
@@ -384,7 +386,8 @@ __device__ int five_point_warp(const double* s1, const double* s2, EmwShared& S,
 }
 
 struct EmatArgs {
-    int n, iters;
+    int n, iters;                          // n < 0: each sequence's count is n_dev[s] (emat_seq reads it)
+    int cap;                               // point slots per sequence
     const float* p1; const float* p2;     // [n][2] pixels
     double fx, fy, cx, cy;
     float thr_sq;
@@ -403,19 +406,38 @@ struct EmatArgs {
     int full;                              // 1: score every sample (the caller reads counts[]); the replay still honours the bound
 };
 
-__global__ void __launch_bounds__(256)
-emat_normalize_kernel(EmatArgs a)
+// the view of sequence s: its slices of every per-sequence array ([cap] points, [iters] samples, 9 doubles of E, 4 ints of
+// result / state, one n and one flag word)
+__device__ __forceinline__ EmatArgs emat_seq(const EmatArgs& A, int s)
 {
+    EmatArgs a = A;
+    const size_t pc = (size_t)s * A.cap, ic = (size_t)s * A.iters;
+    a.p1 += 2 * pc; a.p2 += 2 * pc; a.x1 += 2 * pc; a.x2 += 2 * pc; a.mask += pc;
+    a.samples += 5 * ic; a.models += ic * EM_MAXM * 9; a.nmodels += ic; a.counts += ic * EM_MAXM;
+    a.E += 9 * s; a.result += 4 * s; a.state += 4 * s; a.n_dev += s; a.flags += s;
+    if (A.n < 0) a.n = *a.n_dev;
+    return a;
+}
+
+__global__ void __launch_bounds__(256)
+emat_normalize_kernel(EmatArgs A)
+{
+    const EmatArgs a = emat_seq(A, blockIdx.y);
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i == 0) {   // state: bound, max_good, winner, replayed
+        a.state[0] = a.iters; a.state[1] = 0; a.state[2] = -1; a.state[3] = 0;
+        *a.flags = 0;
+    }
     if (i >= a.n) return;
     a.x1[2 * i] = ((double)a.p1[2 * i] - a.cx) / a.fx; a.x1[2 * i + 1] = ((double)a.p1[2 * i + 1] - a.cy) / a.fy;
     a.x2[2 * i] = ((double)a.p2[2 * i] - a.cx) / a.fx; a.x2[2 * i + 1] = ((double)a.p2[2 * i + 1] - a.cy) / a.fy;
 }
 
 __global__ void __launch_bounds__(EMW_WARPS * 32)
-emat_solve_kernel(EmatArgs a)
+emat_solve_kernel(EmatArgs A)
 {
     __shared__ EmwShared sh[EMW_WARPS];
+    const EmatArgs a = emat_seq(A, blockIdx.y);
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int it = blockIdx.x * EMW_WARPS + warp;
     if (it >= a.iters) return;
@@ -445,10 +467,11 @@ __device__ __forceinline__ bool sampson_inlier(const double* E, double ax, doubl
 
 #define EM_ST 8   // samples per scoring block
 __global__ void __launch_bounds__(256)
-emat_score_kernel(EmatArgs a)
+emat_score_kernel(EmatArgs A)
 {
     __shared__ double s_E[EM_ST * EM_MAXM * 9];
     __shared__ int s_nm[EM_ST];
+    const EmatArgs a = emat_seq(A, blockIdx.z);
     if (!a.full && a.chunk_start >= a.state[0]) return;
     const int it0 = a.chunk_start + blockIdx.y * EM_ST;
     const int ns = min(EM_ST, min(a.iters, a.chunk_start + a.chunk_len) - it0);
@@ -470,9 +493,10 @@ emat_score_kernel(EmatArgs a)
 }
 
 // replay of cv2's sequential loop over this chunk's (sample, model) counts; shrinks the bound
-__global__ void emat_update_kernel(EmatArgs a)
+__global__ void emat_update_kernel(EmatArgs A)
 {
-    if (threadIdx.x != 0 || blockIdx.x != 0) return;
+    if (threadIdx.x != 0) return;
+    const EmatArgs a = emat_seq(A, blockIdx.x);
     int niters = a.state[0], max_good = a.state[1], win = a.state[2];
     if (a.chunk_start >= niters) return;
     const int N = a.n;
@@ -496,9 +520,10 @@ __global__ void emat_update_kernel(EmatArgs a)
 }
 
 __global__ void __launch_bounds__(256)
-emat_finish_kernel(EmatArgs a)
+emat_finish_kernel(EmatArgs A)
 {
     __shared__ double s_E[9];
+    const EmatArgs a = emat_seq(A, blockIdx.x);
     const int win = a.state[2];
     if (threadIdx.x == 0) { a.result[0] = win >= 0; a.result[1] = a.state[3]; a.result[2] = win; }
     if (win < 0) {
@@ -516,12 +541,75 @@ int vo_rng_table(b200vo_ctx* ctx, int n, const uint32_t** d_table);
 // dev_io != nullptr: p1 / p2 are DEVICE pointers and the results go to dev_io (device) instead of E / mask / found
 struct EmatDevIO { double* E; uint8_t* mask; int32_t* found; };
 
-__global__ void emat_export_kernel(EmatArgs a, EmatDevIO io)
+__global__ void emat_export_kernel(EmatArgs A, EmatDevIO io)
 {
+    const EmatArgs a = emat_seq(A, 0);
     const int ok = a.result[0];
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < a.n; i += gridDim.x * blockDim.x) io.mask[i] = ok ? a.mask[i] : 0;
     if (blockIdx.x == 0 && threadIdx.x < 9) io.E[threadIdx.x] = ok ? a.E[threadIdx.x] : 0.0;
     if (blockIdx.x == 0 && threadIdx.x == 0) *io.found = ok;
+}
+
+// Enqueues the RANSAC of `nseq` point sets on the ctx stream; the device arrays of `a` are set, a.n_dev holds each set's
+// point count (at most max_n <= a.cap).  draw: the samples come from cv2's RNG stream (else a.samples is the caller's).
+static int emat_launch(b200vo_ctx* ctx, EmatArgs& a, int nseq, int max_n, bool draw)
+{
+    const int iters = a.iters;
+    const int n_raw = 10 * iters + 256;
+    const int pb = (max_n + 255) / 256 > 0 ? (max_n + 255) / 256 : 1;
+    emat_normalize_kernel<<<dim3(pb, nseq), 256, 0, ctx->stream>>>(a);
+    ctx->launches++;
+    if (draw) {
+        const uint32_t* rng = nullptr;
+        VO_TRY(vo_rng_table(ctx, n_raw, &rng));
+        const size_t smem = (size_t)n_raw * sizeof(int);
+        if (smem > 48 * 1024)
+            VO_CUDA(ctx, cudaFuncSetAttribute(ransac_samples_kernel<5>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        ransac_samples_kernel<5><<<nseq, 128, smem, ctx->stream>>>(rng, n_raw, a.n_dev, iters, a.samples, a.flags);
+        ctx->launches++;
+    }
+    // every sample is solved up front: one warp each, so the launch is one wave of latency-bound warps
+    // whether it carries 128 samples or all of them
+    emat_solve_kernel<<<dim3((iters + EMW_WARPS - 1) / EMW_WARPS, nseq), EMW_WARPS * 32, 0, ctx->stream>>>(a);
+    ctx->launches += 1;
+    // scoring chunks of 64, 128, 256, ... samples: cv2 usually stops within the first (10-60 samples), and every
+    // chunk beyond the bound (known on the device after the previous chunk) costs two empty launches
+    for (int c0 = 0, len = 64; c0 < iters; c0 += len, len *= 2) {
+        a.chunk_start = c0; a.chunk_len = len;
+        emat_score_kernel<<<dim3(pb, (len + EM_ST - 1) / EM_ST, nseq), 256, 0, ctx->stream>>>(a);
+        emat_update_kernel<<<nseq, 32, 0, ctx->stream>>>(a);
+        ctx->launches += 2;
+    }
+    emat_finish_kernel<<<nseq, 256, 0, ctx->stream>>>(a);
+    ctx->launches += 1;
+    VO_CUDA(ctx, cudaGetLastError());
+    return 0;
+}
+
+int vo_emat_batch(b200vo_ctx* ctx, const float* p1, const float* p2, int cap, const int* n_dev, int max_n, int nseq, const double K[9],
+                  double prob, double thr, int max_iters, double* E_dev, uint8_t* mask_dev, int* result_dev, int* flags_dev)
+{
+    const int iters = max_iters > 1 ? max_iters : 1;
+    EmatArgs a{};
+    a.n = -1; a.iters = iters; a.cap = cap;
+    a.fx = K[0]; a.fy = K[4]; a.cx = K[2]; a.cy = K[5];
+    const double t = thr / ((a.fx + a.fy) / 2);
+    a.thr_sq = (float)(t * t);
+    a.conf = prob;
+    const size_t ns = nseq;
+    const size_t b_x = vo_align(ns * cap * 16, 256), b_s = vo_align(ns * iters * 5 * 4, 256), b_m = vo_align(ns * iters * EM_MAXM * 9 * 8, 256);
+    const size_t b_nm = vo_align(ns * iters * 4, 256), b_c = vo_align(ns * iters * EM_MAXM * 4, 256), b_st = vo_align(ns * 16, 256);
+    VO_TRY(vo_reserve(ctx, ctx->d_scratch[5], 2 * b_x + b_s + b_m + b_nm + b_c + b_st));
+    uint8_t* d = (uint8_t*)ctx->d_scratch[5].p;
+    a.p1 = p1; a.p2 = p2; a.n_dev = const_cast<int*>(n_dev);
+    a.x1 = (double*)d; a.x2 = (double*)(d + b_x); d += 2 * b_x;
+    a.samples = (int*)d; d += b_s;
+    a.models = (double*)d; d += b_m;
+    a.nmodels = (int*)d; d += b_nm;
+    a.counts = (int*)d; d += b_c;
+    a.state = (int*)d; a.flags = flags_dev;
+    a.E = E_dev; a.mask = mask_dev; a.result = result_dev;
+    return emat_launch(ctx, a, nseq, max_n, true);
 }
 
 static int emat_run(b200vo_ctx* ctx, const float* p1, const float* p2, int n, const double K[9], const int32_t* samples,
@@ -540,15 +628,12 @@ static int emat_run(b200vo_ctx* ctx, const float* p1, const float* p2, int n, co
     VO_CUDA(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
     const int iters = max_iters > 1 ? max_iters : 1;
     EmatArgs a{};
-    a.n = n; a.iters = iters;
+    a.n = n; a.iters = iters; a.cap = n;
     a.fx = K[0]; a.fy = K[4]; a.cx = K[2]; a.cy = K[5];
     const double t = thr / ((a.fx + a.fy) / 2);
     a.thr_sq = (float)(t * t);
     a.conf = prob;
     a.full = samples != nullptr;
-    const int n_raw = 10 * iters + 256;
-    const uint32_t* rng = nullptr;
-    VO_TRY(vo_rng_table(ctx, n_raw, &rng));
     const size_t b_p = vo_align((size_t)n * 8, 256), b_x = vo_align((size_t)n * 16, 256);
     const size_t b_s = vo_align((size_t)iters * 5 * 4, 256), b_m = vo_align((size_t)iters * EM_MAXM * 9 * 8, 256);
     const size_t b_nm = vo_align((size_t)iters * 4, 256), b_c = vo_align((size_t)iters * EM_MAXM * 4, 256);
@@ -578,37 +663,13 @@ static int emat_run(b200vo_ctx* ctx, const float* p1, const float* p2, int n, co
     VO_CUDA(ctx, cudaMemsetAsync(d_small, 0, 512, ctx->stream));
     int* h_small = (int*)(hp + 2 * b_p + b_mask);
     h_small[0] = n;
-    h_small[1] = iters; h_small[2] = 0; h_small[3] = -1; h_small[4] = 0;   // state: bound, max_good, winner, replayed
     VO_CUDA(ctx, cudaMemcpyAsync(a.n_dev, h_small, 4, cudaMemcpyHostToDevice, ctx->stream));
-    VO_CUDA(ctx, cudaMemcpyAsync(a.state, h_small + 1, 16, cudaMemcpyHostToDevice, ctx->stream));
-    emat_normalize_kernel<<<(n + 255) / 256, 256, 0, ctx->stream>>>(a);
     uint8_t* h_dbg = hp + 2 * b_p + b_mask + 1024;
     if (samples) {   // the caller's sample set (parity runs: same hypotheses as the oracle / as cv2's RNG replay)
         memcpy(h_dbg, samples, (size_t)iters * 5 * 4);
         VO_CUDA(ctx, cudaMemcpyAsync(a.samples, h_dbg, (size_t)iters * 5 * 4, cudaMemcpyHostToDevice, ctx->stream));
-    } else {
-        const size_t smem = (size_t)n_raw * sizeof(int);
-        if (smem > 48 * 1024)
-            VO_CUDA(ctx, cudaFuncSetAttribute(ransac_samples_kernel<5>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        ransac_samples_kernel<5><<<1, 128, smem, ctx->stream>>>(rng, n_raw, a.n_dev, iters, a.samples, a.flags);
     }
-    // chunks of hypotheses in stream order; a chunk whose first sample lies beyond cv2's adaptive
-    // iteration bound (known on the device after the previous chunk) exits immediately
-    ctx->launches += 2;
-    // every sample is solved up front: one warp each, so the launch is one wave of latency-bound warps
-    // whether it carries 128 samples or all of them
-    emat_solve_kernel<<<(iters + EMW_WARPS - 1) / EMW_WARPS, EMW_WARPS * 32, 0, ctx->stream>>>(a);
-    ctx->launches += 1;
-    // scoring chunks of 64, 128, 256, ... samples: cv2 usually stops within the first (10-60 samples), and every
-    // chunk beyond the bound costs two empty launches
-    for (int c0 = 0, len = 64; c0 < iters; c0 += len, len *= 2) {
-        a.chunk_start = c0; a.chunk_len = len;
-        emat_score_kernel<<<dim3((n + 255) / 256, (len + EM_ST - 1) / EM_ST), 256, 0, ctx->stream>>>(a);
-        emat_update_kernel<<<1, 32, 0, ctx->stream>>>(a);
-        ctx->launches += 2;
-    }
-    emat_finish_kernel<<<1, 256, 0, ctx->stream>>>(a);
-    ctx->launches += 1;
+    VO_TRY(emat_launch(ctx, a, 1, n, samples == nullptr));
     VO_CUDA(ctx, cudaGetLastError());
     if (dev_io) {   // results stay on the device; nothing to wait for
         emat_export_kernel<<<(n + 255) / 256, 256, 0, ctx->stream>>>(a, *dev_io);

@@ -67,6 +67,8 @@ struct b200vo_ctx {
     DevBuf d_klt_queue;      // ring of work-queue counters for the persistent tracker kernel
     unsigned klt_queue_next = 0;
     DevBuf d_sift;           // SIFT scale-space workspace (sift.cu)
+    DevBuf d_sift_out[2];    // SIFT keypoints (6 floats a row) and descriptors of the last vo_sift_frames call
+    DevBuf d_sift_sort;      // SIFT keypoint sort scratch
     DevBuf d_rng;            // raw cv::RNG stream (uint32)
     int n_rng = 0;
     // tensor-map encode entry point (driver API, fetched lazily)
@@ -121,3 +123,8 @@ void vo_klt_trace_read(b200vo_ctx* ctx, std::vector<unsigned long long>& out);  
 int vo_klt_launch2(b200vo_ctx* ctx, const PyrGeom& g, const uint8_t* d_prev_slab, size_t prev_stride,
                    const uint8_t* d_next_slab, size_t next_stride, int batch, const KltPointSet* sets, int n_sets,
                    int n_fixed, const KltParams& kp, cudaStream_t stream);
+
+// ---- knn.cu: device-resident kNN(k=2) + ratio test on the ctx stream (descriptors float32 [n][128])
+size_t vo_knn2_workspace(const b200vo_ctx* ctx, int nq, int nt);   // the scratch vo_knn2_ratio_dev reserves
+int vo_knn2_ratio_dev(b200vo_ctx* ctx, const float* q_dev, int nq, const float* t_dev, int nt, double ratio,
+                      int* idx2_dev, float* dist2_dev, uint8_t* accept_dev, int* bad_flag_host);

@@ -399,6 +399,20 @@ static int knn_make_map_ext(b200vo_ctx* ctx, CUtensorMap* map, void* gptr, int r
     return vo_encode_tiled(ctx, map, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, gptr, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_32B);
 }
 
+// scratch of vo_knn2_ratio_dev for nq queries and nt train descriptors (bytes of ctx->d_scratch[3])
+size_t vo_knn2_workspace(const b200vo_ctx* ctx, int nq, int nt)
+{
+    const int nq_pad = (int)vo_align((size_t)nq, 2 * KNN_BM), nt_pad = (int)vo_align((size_t)nt, K3_BN);
+    const int m_pairs = nq_pad / (2 * KNN_BM), n_tiles = nt_pad / K3_BN;
+    const int total = m_pairs * n_tiles;
+    const int per = (total + ctx->num_sms - 1) / ctx->num_sms;
+    const int n_splits = (n_tiles + per - 1) / per + 1;
+    const size_t b_q16 = vo_align((size_t)nq_pad * KNN_DIM * 2, 1024), b_t16 = vo_align((size_t)nt_pad * KNN_DIM * 2, 1024);
+    const size_t b_qx = vo_align((size_t)nq_pad * 32, 1024), b_tx = vo_align((size_t)nt_pad * 32, 1024);
+    const size_t b_part = vo_align((size_t)2 * n_splits * nq_pad * sizeof(KnnPartial), 256);
+    return b_q16 + b_t16 + b_qx + b_tx + b_part + 256;
+}
+
 // device-resident core: q_dev/t_dev float32 row-major; outputs device pointers
 int vo_knn2_ratio_dev(b200vo_ctx* ctx, const float* q_dev, int nq, const float* t_dev, int nt, double ratio,
                       int* idx2_dev, float* dist2_dev, uint8_t* accept_dev, int* bad_flag_host)
@@ -412,7 +426,7 @@ int vo_knn2_ratio_dev(b200vo_ctx* ctx, const float* q_dev, int nq, const float* 
     const size_t b_q16 = vo_align((size_t)nq_pad * KNN_DIM * 2, 1024), b_t16 = vo_align((size_t)nt_pad * KNN_DIM * 2, 1024);
     const size_t b_qx = vo_align((size_t)nq_pad * 32, 1024), b_tx = vo_align((size_t)nt_pad * 32, 1024);
     const size_t b_part = vo_align((size_t)2 * n_splits * nq_pad * sizeof(KnnPartial), 256);
-    VO_TRY(vo_reserve(ctx, ctx->d_scratch[3], b_q16 + b_t16 + b_qx + b_tx + b_part + 256));
+    VO_TRY(vo_reserve(ctx, ctx->d_scratch[3], vo_knn2_workspace(ctx, nq, nt)));
     uint8_t* d = (uint8_t*)ctx->d_scratch[3].p;
     __half* q16 = (__half*)d; d += b_q16;
     __half* t16 = (__half*)d; d += b_t16;

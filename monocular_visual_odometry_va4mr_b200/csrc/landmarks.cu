@@ -412,25 +412,15 @@ extern "C" int b200vo_batch_triangulate_landmarks(b200vo_ctx* ctx, const double 
 }
 
 // ------------------------------------------------------------------------------------------
-// f3: cv2.recoverPose(E, points1, points2, K) at reference :315 (default distanceThresh = 50).
+// f3: cv2.recoverPose(E, points1, points2, K) at reference :315 (default distanceThresh = 50), for a batch of independent
+// (E, point set) pairs; the sequence is taken from the grid and one call is the batch of one.
 //   recover_decompose_kernel   one thread: SVD of E (OpenCV's small-matrix Jacobi), det sign fix,
 //                              R1 = U W Vt, R2 = U W^T Vt, t = U[:,2]; the four [R | +-t]
 //   recover_cheirality_kernel  one thread per (point, pose): 4x4 DLT with P0 = [I|0] on
 //                              K-normalised float64 points, Jacobi SVD, the three sign / depth
 //                              tests -> mask 0 / 255; warp-aggregated counts
-// The winner (most passing points; ties in the order 1, 2, 3, 4) is picked by the host from the
-// four counts -- one 16-byte read the synchronous call needs anyway.
+//   recover_pick_kernel        the winner: most passing points, ties in the order 1, 2, 3, 4
 // ------------------------------------------------------------------------------------------
-struct RecArgs {
-    double E[9];
-    double fx, fy, cx, cy, dist;
-    int n;
-    const float* p1; const float* p2;
-    double* poses;     // [4][12] R | t, then R1, R2, t (21 doubles) for the host
-    uint8_t* masks;    // [4][n]
-    int* good;         // [4]
-};
-
 __device__ __forceinline__ double det3d(const double* M)
 {
     return M[0] * (M[4] * M[8] - M[5] * M[7]) - M[1] * (M[3] * M[8] - M[5] * M[6]) + M[2] * (M[3] * M[7] - M[4] * M[6]);
@@ -445,20 +435,23 @@ __device__ __forceinline__ void mat3_mul(const double* A, const double* B, doubl
 
 __global__ void recover_decompose_kernel(RecArgs a)
 {
-    if (threadIdx.x != 0 || blockIdx.x != 0) return;
-    double W[3], U[9], Vt[9], At[9], T[9], R1[9], R2[9];
-    jacobi_svd<3>(a.E, W, U, Vt, At);
+    const int s = blockIdx.x;
+    if (threadIdx.x != 0 || (a.valid && !a.valid[a.valid_stride * s])) return;
+    double E[9], W[3], U[9], Vt[9], At[9], T[9], R1[9], R2[9];
+    for (int k = 0; k < 9; ++k) E[k] = a.E[9 * s + k];
+    jacobi_svd<3>(E, W, U, Vt, At);
     if (det3d(U) < 0) for (int k = 0; k < 9; ++k) U[k] = -U[k];
     if (det3d(Vt) < 0) for (int k = 0; k < 9; ++k) Vt[k] = -Vt[k];
     const double Wm[9] = {0, 1, 0, -1, 0, 0, 0, 0, 1}, Wt[9] = {0, -1, 0, 1, 0, 0, 0, 0, 1};
     mat3_mul(U, Wm, T); mat3_mul(T, Vt, R1);
     mat3_mul(U, Wt, T); mat3_mul(T, Vt, R2);
     const double t[3] = {U[2], U[5], U[8]};
+    double* poses = a.poses + 48 * s;
     for (int h = 0; h < 4; ++h) {
         const double* R = (h & 1) ? R2 : R1;
         const double sg = h < 2 ? 1.0 : -1.0;
-        for (int k = 0; k < 9; ++k) a.poses[12 * h + k] = R[k];
-        for (int k = 0; k < 3; ++k) a.poses[12 * h + 9 + k] = sg * t[k];
+        for (int k = 0; k < 9; ++k) poses[12 * h + k] = R[k];
+        for (int k = 0; k < 3; ++k) poses[12 * h + 9 + k] = sg * t[k];
     }
 }
 
@@ -466,18 +459,24 @@ __global__ void __launch_bounds__(128)
 recover_cheirality_kernel(RecArgs a)
 {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    const int h = blockIdx.y;
+    const int h = blockIdx.y, s = blockIdx.z;
+    const int n = a.n[s];
+    if (blockIdx.x * blockDim.x >= n) return;
+    const size_t po = (size_t)s * a.cap;
+    const double* poses = a.poses + 48 * s;
     bool ok = false;
-    if (i < a.n) {
+    if (i < n) {
         double P[12];
 #pragma unroll
         for (int r = 0; r < 3; ++r) {
 #pragma unroll
-            for (int c = 0; c < 3; ++c) P[4 * r + c] = a.poses[12 * h + 3 * r + c];
-            P[4 * r + 3] = a.poses[12 * h + 9 + r];
+            for (int c = 0; c < 3; ++c) P[4 * r + c] = poses[12 * h + 3 * r + c];
+            P[4 * r + 3] = poses[12 * h + 9 + r];
         }
-        const double x1 = ((double)a.p1[2 * i] - a.cx) / a.fx, y1 = ((double)a.p1[2 * i + 1] - a.cy) / a.fy;
-        const double x2 = ((double)a.p2[2 * i] - a.cx) / a.fx, y2 = ((double)a.p2[2 * i + 1] - a.cy) / a.fy;
+        const float* p1 = a.p1 + 2 * po;
+        const float* p2 = a.p2 + 2 * po;
+        const double x1 = ((double)p1[2 * i] - a.cx) / a.fx, y1 = ((double)p1[2 * i + 1] - a.cy) / a.fy;
+        const double x2 = ((double)p2[2 * i] - a.cx) / a.fx, y2 = ((double)p2[2 * i + 1] - a.cy) / a.fy;
         double A[16] = {-1, 0, x1, 0, 0, -1, y1, 0, 0, 0, 0, 0, 0, 0, 0, 0}, W[4], U[16], Vt[16], At[16];
 #pragma unroll
         for (int k = 0; k < 4; ++k) { A[8 + k] = x2 * P[8 + k] - P[k]; A[12 + k] = y2 * P[8 + k] - P[4 + k]; }
@@ -488,10 +487,35 @@ recover_cheirality_kernel(RecArgs a)
         ok = ok && (Q2 < a.dist);
         const double z = P[8] * Q0 + P[9] * Q1 + P[10] * Q2 + P[11] * Q3;
         ok = ok && (z > 0) && (z < a.dist);
-        a.masks[(size_t)h * a.n + i] = ok ? 255 : 0;
+        if (a.masks) a.masks[4 * po + (size_t)h * a.cap + i] = ok ? 255 : 0;
     }
     const unsigned bm = __ballot_sync(0xffffffffu, ok);
-    if ((threadIdx.x & 31) == 0 && bm) atomicAdd(a.good + h, __popc(bm));
+    if ((threadIdx.x & 31) == 0 && bm) atomicAdd(a.good + 4 * s + h, __popc(bm));
+}
+
+__global__ void recover_pick_kernel(RecArgs a)
+{
+    const int s = blockIdx.x;
+    if (threadIdx.x != 0) return;
+    const int* good = a.good + 4 * s;
+    int win;
+    if (good[0] >= good[1] && good[0] >= good[2] && good[0] >= good[3]) win = 0;
+    else if (good[1] >= good[0] && good[1] >= good[2] && good[1] >= good[3]) win = 1;
+    else if (good[2] >= good[0] && good[2] >= good[1] && good[2] >= good[3]) win = 2;
+    else win = 3;
+    for (int k = 0; k < 12; ++k) a.Rt[12 * s + k] = a.poses[48 * s + 12 * win + k];
+    a.win[2 * s] = win; a.win[2 * s + 1] = good[win];
+}
+
+int vo_recover_pose_batch_launch(b200vo_ctx* ctx, const RecArgs& a, int nseq, int max_n, cudaStream_t stream)
+{
+    VO_CUDA(ctx, cudaMemsetAsync(a.good, 0, (size_t)nseq * 16, stream));
+    recover_decompose_kernel<<<nseq, 32, 0, stream>>>(a);
+    if (max_n > 0) recover_cheirality_kernel<<<dim3((max_n + 127) / 128, 4, nseq), 128, 0, stream>>>(a);
+    recover_pick_kernel<<<nseq, 32, 0, stream>>>(a);
+    ctx->launches += max_n > 0 ? 3 : 2;
+    VO_CUDA(ctx, cudaGetLastError());
+    return 0;
 }
 
 extern "C" int b200vo_recover_pose(b200vo_ctx* ctx, const double E[9], const float* p1, const float* p2, int n,
@@ -502,41 +526,35 @@ extern "C" int b200vo_recover_pose(b200vo_ctx* ctx, const double E[9], const flo
     VO_CUDA(ctx, cudaSetDevice(ctx->device));
     VO_CUDA(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
     RecArgs a{};
-    for (int k = 0; k < 9; ++k) a.E[k] = E[k];
-    a.fx = K[0]; a.fy = K[4]; a.cx = K[2]; a.cy = K[5]; a.dist = distance_thresh; a.n = n;
+    a.fx = K[0]; a.fy = K[4]; a.cx = K[2]; a.cy = K[5]; a.dist = distance_thresh; a.cap = n;
     const int nn = n > 0 ? n : 1;
     const size_t b_p = vo_align((size_t)nn * 8, 256), b_m = vo_align((size_t)4 * nn, 256), b_small = 512;
-    VO_TRY(vo_reserve(ctx, ctx->d_scratch[7], 2 * b_p + b_m + b_small));
-    VO_TRY(vo_reserve_pinned(ctx, 2 * b_p + b_m + b_small));
+    VO_TRY(vo_reserve(ctx, ctx->d_scratch[7], 2 * b_p + b_small + b_m + b_small));
+    VO_TRY(vo_reserve_pinned(ctx, 2 * b_p + b_small + b_m + b_small));
     uint8_t* d = (uint8_t*)ctx->d_scratch[7].p;
     uint8_t* hp = (uint8_t*)ctx->h_pin;
+    // in: p1 | p2 | E[9], n   out: masks [4][n] | R|t [12], winner, count, good [4] | poses [4][12] (b_small bytes after the masks)
     if (n > 0) { memcpy(hp, p1, (size_t)n * 8); memcpy(hp + b_p, p2, (size_t)n * 8); }
-    VO_CUDA(ctx, cudaMemcpyAsync(d, hp, 2 * b_p, cudaMemcpyHostToDevice, ctx->stream));
+    memcpy(hp + 2 * b_p, E, 72);
+    memcpy(hp + 2 * b_p + 128, &n, 4);
+    VO_CUDA(ctx, cudaMemcpyAsync(d, hp, 2 * b_p + b_small, cudaMemcpyHostToDevice, ctx->stream));
     a.p1 = (const float*)d; a.p2 = (const float*)(d + b_p);
-    a.masks = d + 2 * b_p;
-    a.poses = (double*)(d + 2 * b_p + b_m); a.good = (int*)(d + 2 * b_p + b_m + 384);
-    VO_CUDA(ctx, cudaMemsetAsync(a.poses, 0, b_small, ctx->stream));
-    recover_decompose_kernel<<<1, 32, 0, ctx->stream>>>(a);
-    ctx->launches++;
-    if (n > 0) {
-        recover_cheirality_kernel<<<dim3((n + 127) / 128, 4), 128, 0, ctx->stream>>>(a);
-        ctx->launches++;
-    }
-    VO_CUDA(ctx, cudaGetLastError());
-    VO_CUDA(ctx, cudaMemcpyAsync(hp + 2 * b_p, a.masks, b_m + b_small, cudaMemcpyDeviceToHost, ctx->stream));
+    a.E = (const double*)(d + 2 * b_p); a.n = (const int*)(d + 2 * b_p + 128);
+    uint8_t* dout = d + 2 * b_p + b_small;
+    a.masks = dout;
+    a.Rt = (double*)(dout + b_m); a.win = (int*)(dout + b_m + 96); a.good = (int*)(dout + b_m + 112);
+    a.poses = (double*)(dout + b_m + 128);
+    VO_TRY(vo_recover_pose_batch_launch(ctx, a, 1, n, ctx->stream));
+    uint8_t* ho = hp + 2 * b_p + b_small;
+    VO_CUDA(ctx, cudaMemcpyAsync(ho, dout, b_m + 128, cudaMemcpyDeviceToHost, ctx->stream));
     VO_CUDA(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
     VO_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     cudaEventElapsedTime(&ctx->last_ms, ctx->ev0, ctx->ev1);
-    const double* poses = (const double*)(hp + 2 * b_p + b_m);
-    const int* good = (const int*)(hp + 2 * b_p + b_m + 384);
-    int win;
-    if (good[0] >= good[1] && good[0] >= good[2] && good[0] >= good[3]) win = 0;
-    else if (good[1] >= good[0] && good[1] >= good[2] && good[1] >= good[3]) win = 1;
-    else if (good[2] >= good[0] && good[2] >= good[1] && good[2] >= good[3]) win = 2;
-    else win = 3;
-    for (int k = 0; k < 9; ++k) R[k] = poses[12 * win + k];
-    for (int k = 0; k < 3; ++k) t[k] = poses[12 * win + 9 + k];
-    if (n > 0) memcpy(mask, hp + 2 * b_p + (size_t)win * n, (size_t)n);
-    *n_good = good[win];
+    const double* rt = (const double*)(ho + b_m);
+    const int* w = (const int*)(ho + b_m + 96);
+    for (int k = 0; k < 9; ++k) R[k] = rt[k];
+    for (int k = 0; k < 3; ++k) t[k] = rt[9 + k];
+    if (n > 0) memcpy(mask, ho + (size_t)w[0] * n, (size_t)n);
+    *n_good = w[1];
     return 0;
 }

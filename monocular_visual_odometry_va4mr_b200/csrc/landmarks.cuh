@@ -35,3 +35,21 @@ int vo_triangulate_batch_launch(b200vo_ctx* ctx, const TriBatchArgs& b, int batc
 // min_distance_batch_kernel on `stream` (valid rows >= n[s] are left as they are)
 int vo_min_distance_batch_launch(b200vo_ctx* ctx, int batch, const float* pts, const int* n, int n_cap, const float* existing,
                                  const int* m, int m_cap, float min_dist, uint8_t* valid, cudaStream_t stream);
+
+// cv2.recoverPose for a batch of (E, point set) pairs: sequence s has n[s] <= cap points at p1 / p2 + 2 * s * cap
+struct RecArgs {
+    const double* E;           // [batch][9]
+    const int* valid;          // nullptr or valid[valid_stride * s] != 0: decompose E of sequence s (others keep zero poses)
+    int valid_stride;
+    double fx, fy, cx, cy, dist;
+    int cap;
+    const int* n;              // [batch]
+    const float* p1; const float* p2;
+    double* poses;             // [batch][4][12] R | t of the four decompositions
+    uint8_t* masks;            // nullptr or [batch][4][cap] 0 / 255
+    int* good;                 // [batch][4] points passing the cheirality test
+    double* Rt;                // [batch][12] the winner's R | t
+    int* win;                  // [batch][2] the winner's index and count
+};
+// decompose, cheirality and winner pick on `stream` (max_n >= every n[s]); every pointer of `a` is device memory
+int vo_recover_pose_batch_launch(b200vo_ctx* ctx, const RecArgs& a, int nseq, int max_n, cudaStream_t stream);

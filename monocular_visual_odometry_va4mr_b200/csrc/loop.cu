@@ -6,11 +6,19 @@
 //   commit     stop decisions, inlier landmarks, tracked candidates, (R_CW | t_CW) from rvec | tvec
 //   merge      append the triangulated landmarks, keep the too_short_baseline candidates
 //   append     append the corners that pass the distance filter as candidates, append the pose
+// b200vo_loop_bootstrap runs the reference's `initialization` (:209-245, :295-330) for any subset of the sequences on the device
+// and writes its result straight into the state: batched SIFT (sift.cu), kNN + ratio test per sequence (knn.cu), batched
+// E-RANSAC (emat.cu), batched recoverPose and triangulation (landmarks.cu) and three one-CTA-per-sequence kernels of this file:
+//   boot_match     the ratio-test survivors as (pts0, pts1) pairs, in query order
+//   boot_inliers   the essential-matrix inliers, in order; t * sign(t_z) of the recovered pose
+//   boot_load      capacity decision, the loaded state, the current frame's pyramid, the result block
 // Between steps the state lives in one canonical set of arrays; every kernel that rewrites a range reads it from a
 // scratch copy (the tracker output, the compacted PnP input, the candidates after the status filter), so no kernel
 // reads and writes the same slots.
 #include "batch.cuh"
+#include "emat.cuh"
 #include "landmarks.cuh"
+#include "sift.cuh"
 #include "mathdev.cuh"
 #include "pnp.cuh"
 
@@ -213,6 +221,7 @@ struct b200vo_loop {
     LoopDev d{};
     TriBatchArgs tri{};
     LoopOut res_out{};
+    DevBuf boot_in, boot_ws;     // b200vo_loop_bootstrap: frames and keypoint counts, everything after the matching
 };
 
 extern "C" void b200vo_loop_destroy(b200vo_loop* lp)
@@ -220,7 +229,7 @@ extern "C" void b200vo_loop_destroy(b200vo_loop* lp)
     if (!lp) return;
     cudaSetDevice(lp->ctx->device);
     cudaStreamSynchronize(lp->ctx->stream);
-    for (DevBuf* b : {&lp->mem, &lp->res}) if (b->p) cudaFree(b->p);
+    for (DevBuf* b : {&lp->mem, &lp->res, &lp->boot_in, &lp->boot_ws}) if (b->p) cudaFree(b->p);
     b200vo_batch_destroy(lp->B);
     cudaGetLastError();
     delete lp;
@@ -449,5 +458,256 @@ extern "C" int b200vo_loop_read_state(b200vo_loop* lp, int seq, float* lm, float
     VO_CUDA(ctx, cudaMemcpyAsync(first_pose, d.fpose + co, (size_t)*n_cand * 4, cudaMemcpyDeviceToHost, st));
     VO_CUDA(ctx, cudaMemcpyAsync(poses, d.poses + (size_t)seq * d.P * 12, (size_t)*n_poses * 96, cudaMemcpyDeviceToHost, st));
     VO_CUDA(ctx, cudaStreamSynchronize(st));
+    return 0;
+}
+
+// ------------------------------------------------------------------------------------------
+// bootstrap
+// ------------------------------------------------------------------------------------------
+enum { BT_SEQ, BT_QOFF, BT_NQ, BT_ROW0, BT_ROW1, BT_KINDS };   // per listed sequence, uploaded by the host
+
+struct BootDev {
+    int n_seq, cap;                            // cap: point slots per sequence (most query keypoints of any sequence)
+    const int* tab;                            // [n_seq][BT_KINDS]
+    const float* kp6;                          // SIFT keypoints of every frame (6 floats a row)
+    const int* idx2; const uint8_t* accept;    // kNN of every sequence, rows at its query offset
+    float* pts0; float* pts1; int* n_match;    // [n_seq][cap] ratio-test matches
+    const uint8_t* emask; const int* eres;     // E-RANSAC inlier mask [n_seq][cap], result [n_seq][4] (found first)
+    const int* eflags;                         // E-RANSAC flags [n_seq]: bit 0 = RNG table exhausted
+    float* inl0; float* inl1; int* n_inl;      // the inliers: first_keys, keys
+    const double* Rt;                          // recovered R | t [n_seq][12]
+    double* cur; int* tri_n;                   // current pose (t * sign(t_z)) and the triangulation's point count
+    const uint8_t* keep; const float* new_lm; const float* new_kp; const int* n_new;   // triangulation output
+    const uint8_t* slab; size_t slab_bytes;    // pyramids of frames1 [n_seq]
+    uint8_t* cur_slab;                         // the loop's current-frame slabs [batch]
+    int* res;                                  // [4][n_seq] status | num_pts | n_lm | n_cand
+};
+
+// an essential matrix from cv2's sample stream (a sample draw that ran out of random numbers counts as none found)
+__device__ __forceinline__ bool boot_found(const BootDev& b, int k) { return b.eres[4 * k] != 0 && !(b.eflags[k] & 1); }
+
+__global__ void __launch_bounds__(LOOP_T)
+boot_match_kernel(BootDev b)
+{
+    const int k = blockIdx.x;
+    const int* t = b.tab + BT_KINDS * k;
+    const int qo = t[BT_QOFF], nq = t[BT_NQ];
+    const float* k0 = b.kp6 + (size_t)t[BT_ROW0] * 6;
+    const float* k1 = b.kp6 + (size_t)t[BT_ROW1] * 6;
+    const size_t po = (size_t)k * b.cap;
+    const int n = cta_compact(nq, [&](int i) { return b.accept[qo + i] != 0; },
+                              [&](int i, int o) {
+                                  const int j = b.idx2[2 * (qo + i)];
+                                  b.pts0[2 * (po + o)] = k0[6 * i]; b.pts0[2 * (po + o) + 1] = k0[6 * i + 1];
+                                  b.pts1[2 * (po + o)] = k1[6 * j]; b.pts1[2 * (po + o) + 1] = k1[6 * j + 1];
+                              });
+    if (threadIdx.x == 0) b.n_match[k] = n;
+}
+
+__global__ void __launch_bounds__(LOOP_T)
+boot_inliers_kernel(BootDev b)
+{
+    const int k = blockIdx.x;
+    const bool found = boot_found(b, k);
+    const size_t po = (size_t)k * b.cap;
+    const int n = cta_compact(found ? b.n_match[k] : 0, [&](int i) { return b.emask[po + i] == 1; },
+                              [&](int i, int o) {
+                                  b.inl0[2 * (po + o)] = b.pts0[2 * (po + i)]; b.inl0[2 * (po + o) + 1] = b.pts0[2 * (po + i) + 1];
+                                  b.inl1[2 * (po + o)] = b.pts1[2 * (po + i)]; b.inl1[2 * (po + o) + 1] = b.pts1[2 * (po + i) + 1];
+                              });
+    if (threadIdx.x == 0) b.n_inl[k] = n;
+}
+
+// after recoverPose: the current pose R | t * np.sign(t_z) (:317; sign(0) = 0, sign(NaN) = NaN) and the triangulation's count
+__global__ void boot_pose_kernel(BootDev b)
+{
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= b.n_seq) return;
+    const bool found = boot_found(b, k);
+    const double* rt = b.Rt + 12 * k;
+    const double tz = rt[11];
+    const double sg = tz > 0 ? 1.0 : tz < 0 ? -1.0 : tz == 0 ? 0.0 : tz;
+    for (int q = 0; q < 9; ++q) b.cur[12 * k + q] = rt[q];
+    for (int q = 9; q < 12; ++q) b.cur[12 * k + q] = rt[q] * sg;
+    b.tri_n[k] = found ? b.n_inl[k] : 0;
+}
+
+__global__ void __launch_bounds__(LOOP_T)
+boot_load_kernel(LoopDev d, BootDev b)
+{
+    __shared__ int s_code;
+    const int k = blockIdx.x, tid = threadIdx.x;
+    const int s = b.tab[BT_KINDS * k + BT_SEQ];
+    const size_t po = (size_t)k * b.cap;
+    const bool found = boot_found(b, k);
+    const int n_inl = b.n_inl[k], nn = found ? b.n_new[k] : 0;
+    // the too_short_baseline candidates (keep == 1), counted before anything is written
+    const int nc = cta_compact(found ? n_inl : 0, [&](int i) { return b.keep[po + i] != 0; }, [](int, int) {});
+    if (tid == 0) {
+        s_code = !found ? B200VO_LOOP_NO_BOOTSTRAP : (nn > d.L || nc > d.C) ? B200VO_LOOP_OVERFLOW : B200VO_LOOP_OK;
+        b.res[k] = s_code;
+        b.res[b.n_seq + k] = found ? n_inl : 0;
+        b.res[2 * b.n_seq + k] = s_code == B200VO_LOOP_OK ? nn : 0;
+        b.res[3 * b.n_seq + k] = s_code == B200VO_LOOP_OK ? nc : 0;
+    }
+    __syncthreads();
+    if (s_code != B200VO_LOOP_OK) {   // the state arrays stay as they were; the sequence is skipped until loaded again
+        if (tid == 0) { d.status[s] = s_code; d.trk_lm[s] = 0; d.trk_cand[s] = 0; }
+        return;
+    }
+    const size_t lo = (size_t)s * d.L, co = (size_t)s * d.C;
+    for (int i = tid; i < nn; i += LOOP_T) {
+        d.lm[3 * (lo + i)] = b.new_lm[3 * (po + i)]; d.lm[3 * (lo + i) + 1] = b.new_lm[3 * (po + i) + 1];
+        d.lm[3 * (lo + i) + 2] = b.new_lm[3 * (po + i) + 2];
+        d.lm_kp[2 * (lo + i)] = b.new_kp[2 * (po + i)]; d.lm_kp[2 * (lo + i) + 1] = b.new_kp[2 * (po + i) + 1];
+    }
+    cta_compact(n_inl, [&](int i) { return b.keep[po + i] != 0; },
+                [&](int i, int o) {
+                    d.keys[2 * (co + o)] = b.inl1[2 * (po + i)]; d.keys[2 * (co + o) + 1] = b.inl1[2 * (po + i) + 1];
+                    d.fkeys[2 * (co + o)] = b.inl0[2 * (po + i)]; d.fkeys[2 * (co + o) + 1] = b.inl0[2 * (po + i) + 1];
+                    d.fpose[co + o] = 0;
+                });
+    double* ph = d.poses + (size_t)s * d.P * 12;   // [I | 0], [R | t]
+    if (tid < 12) ph[tid] = (tid == 0 || tid == 4 || tid == 8) ? 1.0 : 0.0;
+    else if (tid < 24) ph[tid] = b.cur[12 * k + tid - 12];
+    const uint4* src = (const uint4*)(b.slab + (size_t)k * b.slab_bytes);
+    uint4* dst = (uint4*)(b.cur_slab + (size_t)s * b.slab_bytes);
+    for (size_t i = tid; i < b.slab_bytes / 16; i += LOOP_T) dst[i] = src[i];
+    if (tid == 0) {
+        d.n_lm[s] = nn; d.n_cand[s] = nc; d.n_poses[s] = 2; d.status[s] = B200VO_LOOP_OK;
+        d.trk_lm[s] = nn; d.trk_cand[s] = nc > 1 ? nc : 0;
+    }
+}
+
+extern "C" int b200vo_loop_bootstrap(b200vo_loop* lp, int n_seq, const int32_t* seqs, const uint8_t* frames0, const uint8_t* frames1,
+                                     double ratio, int32_t* status, int32_t* num_pts, int32_t* n_lm, int32_t* n_cand)
+{
+    if (!lp) return B200VO_E_BADARG;
+    b200vo_ctx* ctx = lp->ctx;
+    b200vo_batch* B = lp->B;
+    if (n_seq < 1 || n_seq > lp->batch) return vo_set_err(ctx, B200VO_E_BADARG, "n_seq = %d is outside [1, batch = %d]", n_seq, lp->batch);
+    if (!seqs || !frames0 || !frames1 || !status || !num_pts || !n_lm || !n_cand) return vo_set_err(ctx, B200VO_E_BADARG, "null array");
+    std::vector<char> seen(lp->batch, 0);
+    for (int k = 0; k < n_seq; ++k) {
+        if (seqs[k] < 0 || seqs[k] >= lp->batch)
+            return vo_set_err(ctx, B200VO_E_BADARG, "seqs[%d] = %d is outside [0, batch = %d)", k, seqs[k], lp->batch);
+        if (seen[seqs[k]]++) return vo_set_err(ctx, B200VO_E_BADARG, "sequence %d is listed twice", seqs[k]);
+    }
+    const int rows = lp->cfg.batch.rows, cols = lp->cfg.batch.cols;
+    const size_t fb = (size_t)rows * cols, sb = B->geom.slab_bytes, ns = n_seq;
+    VO_CUDA(ctx, cudaSetDevice(ctx->device));
+    VO_CUDA(ctx, cudaStreamSynchronize(ctx->stream));   // no step in flight reads the state
+    cudaStream_t st = ctx->stream;
+    // the two frames of sequence k are frames 2k and 2k + 1 of the SIFT batch
+    const size_t b_raw = vo_align(ns * 2 * fb, 256), b_cnt = vo_align(ns * 8, 256);
+    VO_TRY(vo_reserve(ctx, lp->boot_in, b_raw + 2 * b_cnt));
+    uint8_t* raw = (uint8_t*)lp->boot_in.p;
+    int* d_nkp = (int*)(raw + b_raw);
+    int* d_row = (int*)(raw + b_raw + b_cnt);
+    VO_CUDA(ctx, cudaMemcpy2DAsync(raw, 2 * fb, frames0, fb, fb, ns, cudaMemcpyHostToDevice, st));
+    VO_CUDA(ctx, cudaMemcpy2DAsync(raw + fb, 2 * fb, frames1, fb, fb, ns, cudaMemcpyHostToDevice, st));
+    int n_rows = 0;
+    VO_TRY(vo_sift_frames(ctx, raw, fb, 2 * n_seq, rows, cols, true, d_nkp, d_row, &n_rows));
+    std::vector<int> h_cnt(4 * ns);
+    VO_CUDA(ctx, cudaMemcpyAsync(h_cnt.data(), d_nkp, ns * 8, cudaMemcpyDeviceToHost, st));
+    VO_CUDA(ctx, cudaMemcpyAsync(h_cnt.data() + 2 * ns, d_row, ns * 8, cudaMemcpyDeviceToHost, st));
+    VO_CUDA(ctx, cudaStreamSynchronize(st));
+    // per sequence: its query rows, and no matching where knnMatch has no pair to offer (no query descriptors) or the ratio
+    // test cannot run (fewer than two train descriptors)
+    std::vector<int> tab(BT_KINDS * ns);
+    int sum_q = 0, cap = 1;
+    for (int k = 0; k < n_seq; ++k) {
+        const int nq = h_cnt[2 * k], nt = h_cnt[2 * k + 1];
+        int* t = tab.data() + BT_KINDS * k;
+        t[BT_SEQ] = seqs[k]; t[BT_QOFF] = sum_q; t[BT_NQ] = nq > 0 && nt >= 2 ? nq : 0;
+        t[BT_ROW0] = h_cnt[2 * ns + 2 * k]; t[BT_ROW1] = h_cnt[2 * ns + 2 * k + 1];
+        sum_q += t[BT_NQ];
+        cap = std::max(cap, t[BT_NQ]);
+    }
+    const size_t nc = ns * cap, sq = std::max(sum_q, 1);
+    const size_t sizes[] = {ns * BT_KINDS * 4, sq * 8, sq * 8, sq, nc * 8, nc * 8, ns * 4, ns * 72, nc, ns * 16, ns * 4,
+                            nc * 8, nc * 8, ns * 4, nc * 4, ns * 384, ns * 16, ns * 96, ns * 8, ns * 96, ns * 4, ns * 4, ns * 96,
+                            nc, nc * 12, nc * 12, nc * 8, ns * 4, ns * 4, ns * 16, ns * sb};
+    size_t total = 0;
+    for (size_t x : sizes) total += vo_align(x, 256);
+    VO_TRY(vo_reserve(ctx, lp->boot_ws, total));
+    uint8_t* p = (uint8_t*)lp->boot_ws.p;
+    int q = 0;
+    auto take = [&]() { uint8_t* r = p; p += vo_align(sizes[q++], 256); return (void*)r; };
+    BootDev b{};
+    b.n_seq = n_seq; b.cap = cap;
+    int* d_tab = (int*)take();
+    int* idx2 = (int*)take(); float* dist2 = (float*)take(); uint8_t* accept = (uint8_t*)take();
+    b.tab = d_tab; b.idx2 = idx2; b.accept = accept;
+    b.kp6 = (const float*)ctx->d_sift_out[0].p;
+    b.pts0 = (float*)take(); b.pts1 = (float*)take(); b.n_match = (int*)take();
+    double* E = (double*)take(); uint8_t* emask = (uint8_t*)take(); int* eres = (int*)take(); int* eflags = (int*)take();
+    b.emask = emask; b.eres = eres; b.eflags = eflags;
+    b.inl0 = (float*)take(); b.inl1 = (float*)take(); b.n_inl = (int*)take();
+    int* zeros = (int*)take();
+    RecArgs ra{};
+    ra.poses = (double*)take(); ra.good = (int*)take(); ra.Rt = (double*)take(); ra.win = (int*)take();
+    b.Rt = ra.Rt;
+    b.cur = (double*)take(); b.tri_n = (int*)take();
+    int* one = (int*)take();
+    double* first_pose_cw = (double*)take();
+    TriBatchArgs t = lp->tri;
+    t.cap = cap; t.pose_cap = 1;
+    t.keep = (uint8_t*)take(); t.lm_slot = (float*)take(); t.out_lm = (float*)take(); t.out_kp = (float*)take();
+    t.n_new = (int*)take(); t.flags = (int*)take();
+    b.res = (int*)take();
+    uint8_t* slab = (uint8_t*)take();
+    b.keep = t.keep; b.new_lm = t.out_lm; b.new_kp = t.out_kp; b.n_new = t.n_new;
+    b.slab = slab; b.slab_bytes = sb; b.cur_slab = (uint8_t*)B->slabs[B->cur].p;
+    VO_CUDA(ctx, cudaMemcpyAsync(d_tab, tab.data(), ns * BT_KINDS * 4, cudaMemcpyHostToDevice, st));
+    // the triangulation's pose history [I | 0] and every first_pose 0 (:310-313)
+    std::vector<double> id(ns * 12, 0.0);
+    std::vector<int> ones(ns, 1);
+    for (size_t k = 0; k < ns; ++k) id[12 * k] = id[12 * k + 4] = id[12 * k + 8] = 1.0;
+    VO_CUDA(ctx, cudaMemcpyAsync(first_pose_cw, id.data(), ns * 96, cudaMemcpyHostToDevice, st));
+    VO_CUDA(ctx, cudaMemcpyAsync(one, ones.data(), ns * 4, cudaMemcpyHostToDevice, st));
+    VO_CUDA(ctx, cudaMemsetAsync(zeros, 0, nc * 4, st));
+    VO_CUDA(ctx, cudaMemsetAsync(t.flags, 0, ns * 4, st));
+    // kNN(k=2) + ratio test per sequence (query: frame 0, train: frame 1), back to back on the ctx stream, in a workspace
+    // reserved once for the largest of them
+    size_t knn_ws = 0;
+    for (int k = 0; k < n_seq; ++k)
+        if (tab[BT_KINDS * k + BT_NQ] > 0) knn_ws = std::max(knn_ws, vo_knn2_workspace(ctx, tab[BT_KINDS * k + BT_NQ], h_cnt[2 * k + 1]));
+    VO_TRY(vo_reserve(ctx, ctx->d_scratch[3], knn_ws));
+    const float* desc = (const float*)ctx->d_sift_out[1].p;
+    for (int k = 0; k < n_seq; ++k) {
+        const int* tk = tab.data() + BT_KINDS * k;
+        if (tk[BT_NQ] == 0) continue;
+        VO_TRY(vo_knn2_ratio_dev(ctx, desc + (size_t)tk[BT_ROW0] * 128, tk[BT_NQ], desc + (size_t)tk[BT_ROW1] * 128, h_cnt[2 * k + 1], ratio,
+                                 idx2 + 2 * tk[BT_QOFF], dist2 + 2 * tk[BT_QOFF], accept + tk[BT_QOFF], nullptr));
+    }
+    boot_match_kernel<<<n_seq, LOOP_T, 0, st>>>(b);
+    ctx->launches++;
+    // findEssentialMat(RANSAC, prob 0.99, threshold 1.0, maxIters 1000) at :308
+    const double* K = lp->cfg.batch.K;
+    VO_TRY(vo_emat_batch(ctx, b.pts0, b.pts1, cap, b.n_match, cap, n_seq, K, 0.99, 1.0, 1000, E, emask, eres, eflags));
+    boot_inliers_kernel<<<n_seq, LOOP_T, 0, st>>>(b);
+    ctx->launches++;
+    // recoverPose(E, inliers, K) with distanceThresh 50 (:315)
+    ra.E = E; ra.valid = eres; ra.valid_stride = 4;
+    ra.fx = K[0]; ra.fy = K[4]; ra.cx = K[2]; ra.cy = K[5]; ra.dist = 50.0;
+    ra.cap = cap; ra.n = b.n_inl; ra.p1 = b.inl0; ra.p2 = b.inl1;
+    VO_TRY(vo_recover_pose_batch_launch(ctx, ra, n_seq, cap, st));
+    boot_pose_kernel<<<(n_seq + 127) / 128, 128, 0, st>>>(b);
+    ctx->launches++;
+    t.n = b.tri_n; t.n_poses = one; t.cur = b.cur;
+    t.first_keys = b.inl0; t.keys = b.inl1; t.first_pose = zeros; t.poses = first_pose_cw;
+    VO_TRY(vo_triangulate_batch_launch(ctx, t, n_seq, st));
+    VO_TRY(vo_build_pyramids(ctx, raw + fb, 2 * fb, rows, cols, B->geom, slab, sb, n_seq, st));
+    boot_load_kernel<<<n_seq, LOOP_T, 0, st>>>(lp->d, b);
+    ctx->launches++;
+    VO_CUDA(ctx, cudaGetLastError());
+    std::vector<int> h_res(4 * ns);
+    VO_CUDA(ctx, cudaMemcpyAsync(h_res.data(), b.res, ns * 16, cudaMemcpyDeviceToHost, st));
+    VO_CUDA(ctx, cudaStreamSynchronize(st));
+    memcpy(status, h_res.data(), ns * 4);
+    memcpy(num_pts, h_res.data() + ns, ns * 4);
+    memcpy(n_lm, h_res.data() + 2 * ns, ns * 4);
+    memcpy(n_cand, h_res.data() + 3 * ns, ns * 4);
     return 0;
 }

@@ -13,13 +13,17 @@
 //
 // Stages: doubled image -> base blur -> per octave: 5 blurs (row pass, column pass writing the Gaussian image and the DoG
 // image), nearest-neighbour halving -> extrema + refinement (one thread per DoG pixel) -> orientation histograms (one
-// CTA per extremum) -> descriptors (one CTA per keypoint) -> host: cv2's KeyPointsFilter::removeDuplicatedSorted order.
+// CTA per extremum) -> device merge sort in cv2's KeyPointsFilter::removeDuplicatedSorted order and duplicate removal
+// (one CTA per frame) -> descriptors of the ordered list (one CTA per keypoint).
+// Every stage runs for a chunk of same-sized frames at once: the frame index is part of the grid, each frame owns one
+// block of the workspace, extrema and keypoints carry their frame.  One frame is the chunk of one.
 #include "internal.cuh"
+#include "sift.cuh"
 #include <algorithm>
 #include <cfloat>
 #include <climits>
 #include <cmath>
-#include <vector>
+#include <cub/device/device_merge_sort.cuh>
 
 #define SIFT_LAYERS 3
 #define SIFT_IMG_BORDER 5
@@ -34,12 +38,14 @@ struct SiftCand {        // an extremum that survived the refinement
     float x, y, size, response;
     int octave_code;     // cv2's packed octave field, before the firstOctave shift
     int o, layer, r, c;  // pyramid octave index, refined layer, refined integer position
+    int f;               // frame of the chunk
 };
 
 struct SiftKp {          // a keypoint (extremum + one orientation)
     float x, y, size, angle, response;
     int octave_code;
     int o, layer;
+    int f;               // frame of the chunk; -1: a slot freed by the duplicate removal
 };
 
 __device__ __forceinline__ int sift_reflect101(int p, int len)
@@ -53,9 +59,12 @@ __device__ __forceinline__ float sift_exp(float x) { return (float)exp((double)x
 
 // ---------------------------------------------------------------- image doubling (resize INTER_LINEAR, weights 0.25 / 0.75)
 __global__ void __launch_bounds__(256)
-sift_upscale_kernel(const uint8_t* __restrict__ img, int rows, int cols, size_t step, float* __restrict__ out)
+sift_upscale_kernel(const uint8_t* __restrict__ img, int rows, int cols, size_t step, size_t img_stride, float* __restrict__ out,
+                    size_t fstride)
 {
     const int dx = blockIdx.x * blockDim.x + threadIdx.x, dy = blockIdx.y;
+    img += blockIdx.z * img_stride;
+    out += blockIdx.z * fstride;
     if (dx >= 2 * cols) return;
     float fx = (float)((dx + 0.5) * 0.5 - 0.5);
     int sx = sift_floor(fx);
@@ -78,10 +87,12 @@ sift_upscale_kernel(const uint8_t* __restrict__ img, int rows, int cols, size_t 
 // ---------------------------------------------------------------- Gaussian blur, row pass
 #define SIFT_ROW_T 256
 __global__ void __launch_bounds__(SIFT_ROW_T)
-sift_blur_row_kernel(const float* __restrict__ src, float* __restrict__ dst, int rows, int cols, SiftTaps taps)
+sift_blur_row_kernel(const float* __restrict__ src, float* __restrict__ dst, int rows, int cols, SiftTaps taps, size_t fstride)
 {
     __shared__ float s[SIFT_ROW_T + SIFT_MAX_TAPS];
     const int y = blockIdx.y, x0 = blockIdx.x * SIFT_ROW_T, h = taps.n / 2;
+    src += blockIdx.z * fstride;
+    dst += blockIdx.z * fstride;
     const float* row = src + (size_t)y * cols;
     for (int i = threadIdx.x; i < SIFT_ROW_T + 2 * h; i += SIFT_ROW_T) {
         const int x = x0 - h + i;
@@ -104,10 +115,13 @@ sift_blur_row_kernel(const float* __restrict__ src, float* __restrict__ dst, int
 // column pass: writes the Gaussian image and (when prev != nullptr) the DoG image  gauss - prev
 __global__ void __launch_bounds__(256)
 sift_blur_col_kernel(const float* __restrict__ tmp, float* __restrict__ gauss, const float* __restrict__ prev, float* __restrict__ dog,
-                     int rows, int cols, SiftTaps taps)
+                     int rows, int cols, SiftTaps taps, size_t fstride)
 {
     const int x = blockIdx.x * 64 + (threadIdx.x & 63), y = blockIdx.y * 4 + (threadIdx.x >> 6);
     if (x >= cols || y >= rows) return;
+    const size_t fo = blockIdx.z * fstride;
+    tmp += fo; gauss += fo;
+    if (dog) { prev += fo; dog += fo; }
     const int h = taps.n / 2;
     float d = taps.k[h] * tmp[(size_t)y * cols + x];
     const bool fused = x < (cols & ~7);
@@ -121,9 +135,12 @@ sift_blur_col_kernel(const float* __restrict__ tmp, float* __restrict__ gauss, c
 
 // resize(src, Size(cols / 2, rows / 2), INTER_NEAREST): sx = min(floor(x * (1 / (dcols / scols))), scols - 1)
 __global__ void __launch_bounds__(256)
-sift_halve_kernel(const float* __restrict__ src, int srows, int scols, float* __restrict__ dst, int drows, int dcols, double ifx, double ify)
+sift_halve_kernel(const float* __restrict__ src, int srows, int scols, float* __restrict__ dst, int drows, int dcols, double ifx, double ify,
+                  size_t fstride)
 {
     const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y;
+    src += blockIdx.z * fstride;
+    dst += blockIdx.z * fstride;
     if (x >= dcols) return;
     const double fy = y * ify, fx = x * ifx;
     int sy = (int)fy; sy -= (sy > fy); if (sy > srows - 1) sy = srows - 1;
@@ -133,13 +150,14 @@ sift_halve_kernel(const float* __restrict__ src, int srows, int scols, float* __
 
 // ---------------------------------------------------------------- extrema + sub-pixel refinement (adjustLocalExtrema)
 struct SiftOctave {
-    const float* dog[SIFT_LAYERS + 2];
+    const float* dog[SIFT_LAYERS + 2];   // frame 0 of the chunk; frame f at + f * fstride
     int rows, cols, o;
+    size_t fstride;
 };
 
 #define DET2(x, y, z, w) __fmaf_rn((x), (y), -((z) * (w)))
 
-__device__ bool sift_adjust(const SiftOctave& O, int& layer, int& r, int& c, SiftCand& out)
+__device__ bool sift_adjust(const SiftOctave& O, size_t fo, int& layer, int& r, int& c, SiftCand& out)
 {
     const float img_scale = 1.f / 255, deriv_scale = img_scale * 0.5f, second_deriv_scale = img_scale, cross_deriv_scale = img_scale * 0.25f;
     const int cols = O.cols, rows = O.rows;
@@ -147,7 +165,7 @@ __device__ bool sift_adjust(const SiftOctave& O, int& layer, int& r, int& c, Sif
     int i = 0;
 #define AT(im, rr, cc) ((im)[(size_t)(rr) * cols + (cc)])
     for (; i < SIFT_MAX_INTERP_STEPS; ++i) {
-        const float *img = O.dog[layer], *prev = O.dog[layer - 1], *next = O.dog[layer + 1];
+        const float *img = O.dog[layer] + fo, *prev = O.dog[layer - 1] + fo, *next = O.dog[layer + 1] + fo;
         const float b0 = (AT(img, r, c + 1) - AT(img, r, c - 1)) * deriv_scale, b1 = (AT(img, r + 1, c) - AT(img, r - 1, c)) * deriv_scale,
                     b2 = (AT(next, r, c) - AT(prev, r, c)) * deriv_scale;
         const float v2 = AT(img, r, c) * 2;
@@ -182,7 +200,7 @@ __device__ bool sift_adjust(const SiftOctave& O, int& layer, int& r, int& c, Sif
     if (i >= SIFT_MAX_INTERP_STEPS) return false;
     float contr;
     {
-        const float *img = O.dog[layer], *prev = O.dog[layer - 1], *next = O.dog[layer + 1];
+        const float *img = O.dog[layer] + fo, *prev = O.dog[layer - 1] + fo, *next = O.dog[layer + 1] + fo;
         const float b0 = (AT(img, r, c + 1) - AT(img, r, c - 1)) * deriv_scale, b1 = (AT(img, r + 1, c) - AT(img, r - 1, c)) * deriv_scale,
                     b2 = (AT(next, r, c) - AT(prev, r, c)) * deriv_scale;
         const float t = b0 * xc + b1 * xr + b2 * xi;
@@ -211,10 +229,10 @@ __global__ void __launch_bounds__(256)
 sift_extrema_kernel(SiftOctave O, SiftCand* __restrict__ cands, int* __restrict__ n_cands, int cap)
 {
     const int c = SIFT_IMG_BORDER + blockIdx.x * 64 + (threadIdx.x & 63), r = SIFT_IMG_BORDER + blockIdx.y * 4 + (threadIdx.x >> 6);
-    const int layer0 = 1 + blockIdx.z;
+    const int f = blockIdx.z / SIFT_LAYERS, layer0 = 1 + blockIdx.z - f * SIFT_LAYERS;
     if (c >= O.cols - SIFT_IMG_BORDER || r >= O.rows - SIFT_IMG_BORDER) return;
     const int cols = O.cols;
-    const float *img = O.dog[layer0], *prev = O.dog[layer0 - 1], *next = O.dog[layer0 + 1];
+    const float *img = O.dog[layer0] + f * O.fstride, *prev = O.dog[layer0 - 1] + f * O.fstride, *next = O.dog[layer0 + 1] + f * O.fstride;
     const float val = img[(size_t)r * cols + c];
     if (!(fabsf(val) > 1.f)) return;      // threshold = cvFloor(0.5 * 0.04 / 3 * 255) = 1
     bool ext = true;
@@ -238,7 +256,8 @@ sift_extrema_kernel(SiftOctave O, SiftCand* __restrict__ cands, int* __restrict_
     if (!ext) return;
     SiftCand cd;
     int layer = layer0, r1 = r, c1 = c;
-    if (!sift_adjust(O, layer, r1, c1, cd)) return;
+    if (!sift_adjust(O, f * O.fstride, layer, r1, c1, cd)) return;
+    cd.f = f;
     const int slot = atomicAdd(n_cands, 1);
     if (slot < cap) cands[slot] = cd;
 }
@@ -260,8 +279,9 @@ __device__ __forceinline__ float sift_fast_atan2(float y, float x)
 }
 
 struct SiftPyrDev {
-    const float* gauss[SIFT_MAX_OCTAVES][SIFT_LAYERS + 3];
+    const float* gauss[SIFT_MAX_OCTAVES][SIFT_LAYERS + 3];   // frame 0 of the chunk; frame f at + f * fstride
     int rows[SIFT_MAX_OCTAVES], cols[SIFT_MAX_OCTAVES];
+    size_t fstride;
 };
 
 #define SIFT_ORI_T 128
@@ -276,7 +296,7 @@ sift_orientation_kernel(SiftPyrDev P, const SiftCand* __restrict__ cands, int n_
     if (ci >= n_cands) return;
     const SiftCand cd = cands[ci];
     const int o = cd.o, rows = P.rows[o], cols = P.cols[o], n = SIFT_ORI_BINS;
-    const float* img = P.gauss[o][cd.layer];
+    const float* img = P.gauss[o][cd.layer] + cd.f * P.fstride;
     const float scl_octv = cd.size * 0.5f / (1 << o);
     const int radius = __float2int_rn(4.5f * scl_octv);
     const float sigma = 1.5f * scl_octv;
@@ -339,7 +359,7 @@ sift_orientation_kernel(SiftPyrDev P, const SiftCand* __restrict__ cands, int n_
             if (slot < cap) {
                 SiftKp kp;
                 kp.x = cd.x; kp.y = cd.y; kp.size = cd.size; kp.angle = angle; kp.response = cd.response;
-                kp.octave_code = cd.octave_code; kp.o = cd.o; kp.layer = cd.layer;
+                kp.octave_code = cd.octave_code; kp.o = cd.o; kp.layer = cd.layer; kp.f = cd.f;
                 kps[slot] = kp;
             }
         }
@@ -354,7 +374,7 @@ sift_orientation_kernel(SiftPyrDev P, const SiftCand* __restrict__ cands, int n_
 
 __global__ void __launch_bounds__(SIFT_DESC_T)
 sift_descriptor_kernel(SiftPyrDev P, const SiftKp* __restrict__ kps, int n_kps, float* __restrict__ desc)
-{
+{   // kps: the ordered, deduplicated list with the freed slots marked f = -1; row ki of desc belongs to kps[ki]
     __shared__ float s_hist[SIFT_HIST];
     __shared__ float s_v[8][SIFT_DESC_T];
     __shared__ int s_cell[SIFT_DESC_T];        // ((r0 + 1) * 6 + (c0 + 1)) * 16 + o0 of the compacted valid samples, in raster order
@@ -364,6 +384,7 @@ sift_descriptor_kernel(SiftPyrDev P, const SiftKp* __restrict__ kps, int n_kps, 
     const int ki = blockIdx.x;
     if (ki >= n_kps) return;
     const SiftKp kp = kps[ki];
+    if (kp.f < 0) return;
     const int d = SIFT_D, n = SIFT_N;
     // detectAndCompute: kpt.octave / pt / size are shifted by firstOctave = -1 before the descriptors; unpackOctave then scales
     // them back to the octave's own resolution.  In pyramid-index terms: scale = 1 / 2^o applied to the unshifted values,
@@ -376,7 +397,7 @@ sift_descriptor_kernel(SiftPyrDev P, const SiftKp* __restrict__ kps, int n_kps, 
     if (fabsf(ori - 360.f) < FLT_EPSILON) ori = 0.f;
     const float scl = size * 0.5f;
     const int rows = P.rows[o], cols = P.cols[o];
-    const float* img = P.gauss[o][kp.layer];
+    const float* img = P.gauss[o][kp.layer] + kp.f * P.fstride;
     const int px = __float2int_rn(ptx), py = __float2int_rn(pty);
     float cos_t = (float)cos((double)(ori * (float)(3.14159265358979323846 / 180)));
     float sin_t = (float)sin((double)(ori * (float)(3.14159265358979323846 / 180)));
@@ -487,6 +508,82 @@ sift_descriptor_kernel(SiftPyrDev P, const SiftKp* __restrict__ kps, int n_kps, 
     }
 }
 
+// ---------------------------------------------------------------- cv2's keypoint order, duplicate removal
+// KeyPointsFilter::removeDuplicatedSorted (features2d/src/keypoint.cpp) sorts by (x, y, -size, angle, -response, -octave) and
+// drops every keypoint equal in (x, y, size, angle) to the one before it.  The frame comes first, so one sort orders every
+// frame of a chunk.  Keypoints equal in all six fields are identical (descriptor included), so their order is immaterial.
+struct SiftKpLess {
+    __device__ __forceinline__ bool operator()(const SiftKp& a, const SiftKp& b) const
+    {
+        if (a.f != b.f) return a.f < b.f;
+        if (a.x != b.x) return a.x < b.x;
+        if (a.y != b.y) return a.y < b.y;
+        if (a.size != b.size) return a.size > b.size;
+        if (a.angle != b.angle) return a.angle < b.angle;
+        if (a.response != b.response) return a.response > b.response;
+        return a.octave_code > b.octave_code;
+    }
+};
+
+#define SIFT_DEDUP_T 256
+// One CTA per frame of the chunk: the frame's run [lo, hi) of the sorted list, first of each (x, y, size, angle) group kept in
+// order (ballot + running base) at out[lo + rank]; the rest of the run is marked free.  Writes the kept keypoints in the
+// caller's format (firstOctave = -1 undone: coordinates and size halved, octave - 1 in the low byte) at kp6[base + lo + rank],
+// and per frame the count and the first row.
+__global__ void __launch_bounds__(SIFT_DEDUP_T)
+sift_dedup_kernel(const SiftKp* __restrict__ sorted, int n, SiftKp* __restrict__ out, float* __restrict__ kp6, int base,
+                  int* __restrict__ n_frame, int* __restrict__ first_row)
+{
+    __shared__ int s_warp[SIFT_DEDUP_T / 32];
+    __shared__ int s_lo, s_hi, s_base;
+    const int f = blockIdx.x, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    if (threadIdx.x < 2) {   // lower bounds of f and f + 1
+        const int key = f + threadIdx.x;
+        int a = 0, b = n;
+        while (a < b) { const int m = (a + b) >> 1; if (sorted[m].f < key) a = m + 1; else b = m; }
+        if (threadIdx.x == 0) s_lo = a; else s_hi = a;
+    }
+    if (threadIdx.x == 0) s_base = 0;
+    __syncthreads();
+    const int lo = s_lo, hi = s_hi;
+    for (int i0 = lo; i0 < hi; i0 += SIFT_DEDUP_T) {
+        const int i = i0 + threadIdx.x;
+        bool keep = false;
+        SiftKp k{};
+        if (i < hi) {
+            k = sorted[i];
+            keep = i == lo;
+            if (!keep) {
+                const SiftKp& p = sorted[i - 1];
+                keep = p.x != k.x || p.y != k.y || p.size != k.size || p.angle != k.angle;
+            }
+        }
+        const unsigned bm = __ballot_sync(0xffffffffu, keep);
+        if (lane == 0) s_warp[warp] = __popc(bm);
+        __syncthreads();
+        int o = s_base;
+        for (int w = 0; w < warp; ++w) o += s_warp[w];
+        o += __popc(bm & ((1u << lane) - 1));
+        if (keep) {
+            out[lo + o] = k;
+            const int oc = (k.octave_code & ~255) | ((k.octave_code - 1) & 255);
+            float* q = kp6 + (size_t)(base + lo + o) * 6;
+            q[0] = k.x * 0.5f; q[1] = k.y * 0.5f; q[2] = k.size * 0.5f; q[3] = k.angle; q[4] = k.response;
+            memcpy(&q[5], &oc, 4);
+        }
+        __syncthreads();
+        if (threadIdx.x == 0) {
+            int tot = 0;
+            for (int w = 0; w < SIFT_DEDUP_T / 32; ++w) tot += s_warp[w];
+            s_base += tot;
+        }
+        __syncthreads();
+    }
+    const int cnt = s_base;
+    for (int i = lo + cnt + threadIdx.x; i < hi; i += SIFT_DEDUP_T) out[i].f = -1;
+    if (threadIdx.x == 0) { n_frame[f] = cnt; first_row[f] = base + lo; }
+}
+
 // ---------------------------------------------------------------- host
 static int sift_kernel_taps(double sigma, SiftTaps* t)
 {
@@ -507,60 +604,81 @@ static int sift_kernel_taps(double sigma, SiftTaps* t)
     return 0;
 }
 
-static int sift_blur(b200vo_ctx* ctx, const float* src, float* tmp, float* gauss, const float* prev, float* dog, int rows, int cols, double sigma)
+static int sift_blur(b200vo_ctx* ctx, const float* src, float* tmp, float* gauss, const float* prev, float* dog, int rows, int cols, double sigma,
+                     int nf, size_t fstride)
 {
     SiftTaps t;
     if (sift_kernel_taps(sigma, &t)) return vo_set_err(ctx, B200VO_E_UNSUPPORTED, "Gaussian kernel of sigma %g needs more than %d taps", sigma, SIFT_MAX_TAPS);
-    sift_blur_row_kernel<<<dim3((cols + SIFT_ROW_T - 1) / SIFT_ROW_T, rows), SIFT_ROW_T, 0, ctx->stream>>>(src, tmp, rows, cols, t);
-    sift_blur_col_kernel<<<dim3((cols + 63) / 64, (rows + 3) / 4), 256, 0, ctx->stream>>>(tmp, gauss, prev, dog, rows, cols, t);
+    sift_blur_row_kernel<<<dim3((cols + SIFT_ROW_T - 1) / SIFT_ROW_T, rows, nf), SIFT_ROW_T, 0, ctx->stream>>>(src, tmp, rows, cols, t, fstride);
+    sift_blur_col_kernel<<<dim3((cols + 63) / 64, (rows + 3) / 4, nf), 256, 0, ctx->stream>>>(tmp, gauss, prev, dog, rows, cols, t, fstride);
     ctx->launches += 2;
     return 0;
 }
 
-struct SiftHostKp { float x, y, size, angle, response; int octave; int src; };
+// Scale space of one frame: the doubled image, the row-pass scratch and per octave 6 Gaussian + 5 DoG images.  Octaves whose
+// images have fewer than 11 rows or columns cannot hold an extremum (5-pixel border) and are not built.
+struct SiftGeom {
+    int brows, bcols, n_act;
+    int orows[SIFT_MAX_OCTAVES], ocols[SIFT_MAX_OCTAVES];
+    size_t o_up, o_tmp, o_g[SIFT_MAX_OCTAVES][SIFT_LAYERS + 3], o_d[SIFT_MAX_OCTAVES][SIFT_LAYERS + 2];
+    size_t frame_bytes;
+};
 
-extern "C" int b200vo_sift_detect_and_compute(b200vo_ctx* ctx, const uint8_t* img, int rows, int cols, size_t step, int max_kp,
-                                              float* kps_out, float* desc_out, int32_t* n_out)
+static void sift_geom(int rows, int cols, SiftGeom& G)
 {
-    if (!ctx || !img || !n_out || rows <= 0 || cols <= 0 || step < (size_t)cols || max_kp < 0 || (max_kp > 0 && !kps_out))
-        return B200VO_E_BADARG;
-    *n_out = 0;
-    VO_CUDA(ctx, cudaSetDevice(ctx->device));
-    VO_CUDA(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
-    const int L = SIFT_LAYERS;
-    const int brows = rows * 2, bcols = cols * 2;
-    const int mn = bcols < brows ? bcols : brows;
+    G.brows = rows * 2; G.bcols = cols * 2;
+    const int mn = G.bcols < G.brows ? G.bcols : G.brows;
     int n_oct = (int)lrint(log((double)mn) / log(2.) - 2) + 1;       // firstOctave = -1
     if (n_oct < 1) n_oct = 1;
-    // octaves whose images have fewer than 11 rows or columns cannot hold an extremum (5-pixel border): not built
-    int orows[SIFT_MAX_OCTAVES], ocols[SIFT_MAX_OCTAVES], n_act = 0;
-    for (int o = 0, r = brows, c = bcols; o < n_oct && o < SIFT_MAX_OCTAVES; ++o, r /= 2, c /= 2) {
+    G.n_act = 0;
+    for (int o = 0, r = G.brows, c = G.bcols; o < n_oct && o < SIFT_MAX_OCTAVES; ++o, r /= 2, c /= 2) {
         if (r < 2 * SIFT_IMG_BORDER + 1 || c < 2 * SIFT_IMG_BORDER + 1) break;
-        orows[o] = r; ocols[o] = c; n_act = o + 1;
+        G.orows[o] = r; G.ocols[o] = c; G.n_act = o + 1;
     }
-    const int cand_cap = 1 << 18, kp_cap = 1 << 18;
-    // workspace: raw image | doubled image | row-pass scratch | per octave 6 Gaussian + 5 DoG images | candidates | keypoints | counters
     size_t off = 0;
     auto take = [&](size_t bytes) { const size_t o2 = off; off += vo_align(bytes, 256); return o2; };
-    const size_t base_px = (size_t)brows * bcols;
-    const size_t o_raw = take((size_t)rows * cols), o_up = take(base_px * 4), o_tmp = take(base_px * 4);
-    size_t o_g[SIFT_MAX_OCTAVES][SIFT_LAYERS + 3], o_d[SIFT_MAX_OCTAVES][SIFT_LAYERS + 2];
-    for (int o = 0; o < n_act; ++o) {
-        const size_t px = (size_t)orows[o] * ocols[o];
-        for (int i = 0; i < L + 3; ++i) o_g[o][i] = take(px * 4);
-        for (int i = 0; i < L + 2; ++i) o_d[o][i] = take(px * 4);
+    const size_t base_px = (size_t)G.brows * G.bcols;
+    G.o_up = take(base_px * 4); G.o_tmp = take(base_px * 4);
+    for (int o = 0; o < G.n_act; ++o) {
+        const size_t px = (size_t)G.orows[o] * G.ocols[o];
+        for (int i = 0; i < SIFT_LAYERS + 3; ++i) G.o_g[o][i] = take(px * 4);
+        for (int i = 0; i < SIFT_LAYERS + 2; ++i) G.o_d[o][i] = take(px * 4);
     }
-    const size_t o_cand = take((size_t)cand_cap * sizeof(SiftCand)), o_kp = take((size_t)kp_cap * sizeof(SiftKp)), o_cnt = take(256);
-    VO_TRY(vo_reserve(ctx, ctx->d_sift, off));
-    uint8_t* ws = (uint8_t*)ctx->d_sift.p;
-    int* d_cnt = (int*)(ws + o_cnt);
-    VO_CUDA(ctx, cudaMemsetAsync(d_cnt, 0, 8, ctx->stream));
-    // upload (tight rows)
-    VO_CUDA(ctx, cudaMemcpy2DAsync(ws + o_raw, cols, img, step, cols, rows, cudaMemcpyHostToDevice, ctx->stream));
-    float* up = (float*)(ws + o_up);
-    float* tmp = (float*)(ws + o_tmp);
-    sift_upscale_kernel<<<dim3((bcols + 255) / 256, brows), 256, 0, ctx->stream>>>(ws + o_raw, rows, cols, (size_t)cols, up);
-    ctx->launches++;
+    G.frame_bytes = off;
+}
+
+#define SIFT_CAND_CAP (1 << 18)    // extrema per frame
+#define SIFT_KP_CAP (1 << 18)      // keypoints per frame
+// The workspace of one chunk of frames, with the quarter vo_reserve adds, fits this budget (about 150 MB per KITTI-sized
+// frame with its extrema and keypoints: 21 frames).
+#define SIFT_CHUNK_BYTES ((size_t)4 << 30)
+
+static size_t sift_per_frame_bytes(const SiftGeom& G)
+{
+    return G.frame_bytes + (size_t)SIFT_CAND_CAP * sizeof(SiftCand) + (size_t)2 * SIFT_KP_CAP * sizeof(SiftKp);
+}
+
+// grows b to `bytes`, keeping its first `used` bytes
+static int sift_reserve_keep(b200vo_ctx* ctx, DevBuf& b, size_t used, size_t bytes)
+{
+    if (bytes <= b.cap) return 0;
+    DevBuf nb;
+    VO_TRY(vo_reserve(ctx, nb, bytes));
+    if (used) VO_CUDA(ctx, cudaMemcpyAsync(nb.p, b.p, used, cudaMemcpyDeviceToDevice, ctx->stream));
+    VO_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    if (b.p) VO_CUDA(ctx, cudaFree(b.p));
+    b = nb;
+    return 0;
+}
+
+int vo_sift_frames(b200vo_ctx* ctx, const uint8_t* d_raw, size_t raw_stride, int n_frames, int rows, int cols, bool want_desc,
+                   int* d_n_frame, int* d_first_row, int* n_rows)
+{
+    const int L = SIFT_LAYERS;
+    SiftGeom G;
+    sift_geom(rows, cols, G);
+    const size_t per_frame = sift_per_frame_bytes(G);
+    const int chunk = (int)std::max<size_t>(1, SIFT_CHUNK_BYTES / 5 * 4 / per_frame);
     double sig[SIFT_LAYERS + 3];
     sig[0] = 1.6;
     const double kk = pow(2., 1. / L);
@@ -570,93 +688,128 @@ extern "C" int b200vo_sift_detect_and_compute(b200vo_ctx* ctx, const uint8_t* im
     }
     const float sg = 1.6f;
     const float sig_diff = sqrtf(std::max(sg * sg - 0.5f * 0.5f * 4, 0.01f));     // createInitialImage: float arithmetic
-    SiftPyrDev P{};
-    for (int o = 0; o < n_act; ++o) {
-        P.rows[o] = orows[o]; P.cols[o] = ocols[o];
-        for (int i = 0; i < L + 3; ++i) P.gauss[o][i] = (const float*)(ws + o_g[o][i]);
-    }
-    for (int o = 0; o < n_act; ++o) {
-        float* g0 = (float*)(ws + o_g[o][0]);
-        if (o == 0) {
-            VO_TRY(sift_blur(ctx, up, tmp, g0, nullptr, nullptr, brows, bcols, (double)sig_diff));
-        } else {
-            const double ifx = 1.0 / ((double)ocols[o] / ocols[o - 1]), ify = 1.0 / ((double)orows[o] / orows[o - 1]);
-            sift_halve_kernel<<<dim3((ocols[o] + 255) / 256, orows[o]), 256, 0, ctx->stream>>>((const float*)(ws + o_g[o - 1][L]), orows[o - 1],
-                                                                                                 ocols[o - 1], g0, orows[o], ocols[o], ifx, ify);
+    const size_t fs = G.frame_bytes / 4;   // frame stride of the workspace, in floats
+    int base = 0;                          // output rows written so far
+    for (int f0 = 0; f0 < n_frames; f0 += chunk) {
+        const int nf = std::min(chunk, n_frames - f0);
+        const size_t cand_cap = (size_t)nf * SIFT_CAND_CAP, kp_cap = (size_t)nf * SIFT_KP_CAP;
+        const size_t o_cand = vo_align((size_t)nf * G.frame_bytes, 256), o_kp = o_cand + vo_align(cand_cap * sizeof(SiftCand), 256);
+        const size_t o_sorted = o_kp + vo_align(kp_cap * sizeof(SiftKp), 256), o_cnt = o_sorted + vo_align(kp_cap * sizeof(SiftKp), 256);
+        VO_TRY(vo_reserve(ctx, ctx->d_sift, o_cnt + 256));
+        uint8_t* ws = (uint8_t*)ctx->d_sift.p;
+        int* d_cnt = (int*)(ws + o_cnt);
+        VO_CUDA(ctx, cudaMemsetAsync(d_cnt, 0, 8, ctx->stream));
+        float* up = (float*)(ws + G.o_up);
+        float* tmp = (float*)(ws + G.o_tmp);
+        sift_upscale_kernel<<<dim3((G.bcols + 255) / 256, G.brows, nf), 256, 0, ctx->stream>>>(d_raw + (size_t)f0 * raw_stride, rows, cols,
+                                                                                              (size_t)cols, raw_stride, up, fs);
+        ctx->launches++;
+        SiftPyrDev P{};
+        P.fstride = fs;
+        for (int o = 0; o < G.n_act; ++o) {
+            P.rows[o] = G.orows[o]; P.cols[o] = G.ocols[o];
+            for (int i = 0; i < L + 3; ++i) P.gauss[o][i] = (const float*)(ws + G.o_g[o][i]);
+        }
+        for (int o = 0; o < G.n_act; ++o) {
+            float* g0 = (float*)(ws + G.o_g[o][0]);
+            if (o == 0) {
+                VO_TRY(sift_blur(ctx, up, tmp, g0, nullptr, nullptr, G.brows, G.bcols, (double)sig_diff, nf, fs));
+            } else {
+                const double ifx = 1.0 / ((double)G.ocols[o] / G.ocols[o - 1]), ify = 1.0 / ((double)G.orows[o] / G.orows[o - 1]);
+                sift_halve_kernel<<<dim3((G.ocols[o] + 255) / 256, G.orows[o], nf), 256, 0, ctx->stream>>>(
+                    (const float*)(ws + G.o_g[o - 1][L]), G.orows[o - 1], G.ocols[o - 1], g0, G.orows[o], G.ocols[o], ifx, ify, fs);
+                ctx->launches++;
+            }
+            for (int i = 1; i < L + 3; ++i)
+                VO_TRY(sift_blur(ctx, (const float*)(ws + G.o_g[o][i - 1]), tmp, (float*)(ws + G.o_g[o][i]), (const float*)(ws + G.o_g[o][i - 1]),
+                                 (float*)(ws + G.o_d[o][i - 1]), G.orows[o], G.ocols[o], sig[i], nf, fs));
+            SiftOctave O{};
+            for (int i = 0; i < L + 2; ++i) O.dog[i] = (const float*)(ws + G.o_d[o][i]);
+            O.rows = G.orows[o]; O.cols = G.ocols[o]; O.o = o; O.fstride = fs;
+            const int ew = G.ocols[o] - 2 * SIFT_IMG_BORDER, eh = G.orows[o] - 2 * SIFT_IMG_BORDER;
+            sift_extrema_kernel<<<dim3((ew + 63) / 64, (eh + 3) / 4, nf * L), 256, 0, ctx->stream>>>(O, (SiftCand*)(ws + o_cand), d_cnt,
+                                                                                                    (int)cand_cap);
             ctx->launches++;
         }
-        for (int i = 1; i < L + 3; ++i)
-            VO_TRY(sift_blur(ctx, (const float*)(ws + o_g[o][i - 1]), tmp, (float*)(ws + o_g[o][i]), (const float*)(ws + o_g[o][i - 1]),
-                             (float*)(ws + o_d[o][i - 1]), orows[o], ocols[o], sig[i]));
-        SiftOctave O{};
-        for (int i = 0; i < L + 2; ++i) O.dog[i] = (const float*)(ws + o_d[o][i]);
-        O.rows = orows[o]; O.cols = ocols[o]; O.o = o;
-        const int ew = ocols[o] - 2 * SIFT_IMG_BORDER, eh = orows[o] - 2 * SIFT_IMG_BORDER;
-        sift_extrema_kernel<<<dim3((ew + 63) / 64, (eh + 3) / 4, L), 256, 0, ctx->stream>>>(O, (SiftCand*)(ws + o_cand), d_cnt, cand_cap);
-        ctx->launches++;
-    }
-    VO_CUDA(ctx, cudaGetLastError());
-    int h_cnt[2] = {0, 0};
-    VO_CUDA(ctx, cudaMemcpyAsync(h_cnt, d_cnt, 4, cudaMemcpyDeviceToHost, ctx->stream));
-    VO_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    if (h_cnt[0] > cand_cap) return vo_set_err(ctx, B200VO_E_UNSUPPORTED, "%d scale-space extrema exceed the limit of %d", h_cnt[0], cand_cap);
-    int n_kp = 0;
-    if (h_cnt[0] > 0) {
-        sift_orientation_kernel<<<h_cnt[0], SIFT_ORI_T, 0, ctx->stream>>>(P, (const SiftCand*)(ws + o_cand), h_cnt[0], (SiftKp*)(ws + o_kp), d_cnt + 1, kp_cap);
-        ctx->launches++;
         VO_CUDA(ctx, cudaGetLastError());
-        VO_CUDA(ctx, cudaMemcpyAsync(h_cnt + 1, d_cnt + 1, 4, cudaMemcpyDeviceToHost, ctx->stream));
+        VO_TRY(vo_reserve_pinned(ctx, 256));
+        int* h_cnt = (int*)ctx->h_pin;
+        VO_CUDA(ctx, cudaMemcpyAsync(h_cnt, d_cnt, 4, cudaMemcpyDeviceToHost, ctx->stream));
         VO_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-        n_kp = h_cnt[1];
-        if (n_kp > kp_cap) return vo_set_err(ctx, B200VO_E_UNSUPPORTED, "%d keypoints exceed the limit of %d", n_kp, kp_cap);
-    }
-    std::vector<SiftKp> hk((size_t)n_kp);
-    std::vector<float> hd;
-    if (n_kp > 0) {
-        VO_CUDA(ctx, cudaMemcpyAsync(hk.data(), ws + o_kp, (size_t)n_kp * sizeof(SiftKp), cudaMemcpyDeviceToHost, ctx->stream));
-        if (desc_out) {
-            // descriptors of the unsorted list go to the (now free) doubled-image + scratch area when they fit, else to their own block
-            const size_t need = (size_t)n_kp * 128 * 4;
-            float* d_desc = nullptr;
-            if (need <= vo_align(base_px * 4, 256) * 2) d_desc = up;
-            else { VO_TRY(vo_reserve(ctx, ctx->d_scratch[4], need)); d_desc = (float*)ctx->d_scratch[4].p; }
-            sift_descriptor_kernel<<<n_kp, SIFT_DESC_T, 0, ctx->stream>>>(P, (const SiftKp*)(ws + o_kp), n_kp, d_desc);
+        const int n_cand = h_cnt[0];
+        if ((size_t)n_cand > cand_cap) return vo_set_err(ctx, B200VO_E_UNSUPPORTED, "%d scale-space extrema exceed the limit of %zu", n_cand, cand_cap);
+        int n_kp = 0;
+        if (n_cand > 0) {
+            sift_orientation_kernel<<<n_cand, SIFT_ORI_T, 0, ctx->stream>>>(P, (const SiftCand*)(ws + o_cand), n_cand, (SiftKp*)(ws + o_kp), d_cnt + 1,
+                                                                           (int)kp_cap);
             ctx->launches++;
             VO_CUDA(ctx, cudaGetLastError());
-            hd.resize((size_t)n_kp * 128);
-            VO_CUDA(ctx, cudaMemcpyAsync(hd.data(), d_desc, need, cudaMemcpyDeviceToHost, ctx->stream));
+            VO_CUDA(ctx, cudaMemcpyAsync(h_cnt + 1, d_cnt + 1, 4, cudaMemcpyDeviceToHost, ctx->stream));
+            VO_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+            n_kp = h_cnt[1];
+            if ((size_t)n_kp > kp_cap) return vo_set_err(ctx, B200VO_E_UNSUPPORTED, "%d keypoints exceed the limit of %zu", n_kp, kp_cap);
         }
+        SiftKp* kps = (SiftKp*)(ws + o_kp);
+        SiftKp* sorted = (SiftKp*)(ws + o_sorted);
+        VO_TRY(sift_reserve_keep(ctx, ctx->d_sift_out[0], (size_t)base * 24, (size_t)(base + n_kp) * 24 + 256));
+        if (want_desc) VO_TRY(sift_reserve_keep(ctx, ctx->d_sift_out[1], (size_t)base * 512, (size_t)(base + n_kp) * 512 + 256));
+        if (n_kp > 0) {
+            size_t tb = 0;
+            VO_CUDA(ctx, cub::DeviceMergeSort::SortKeysCopy(nullptr, tb, kps, sorted, n_kp, SiftKpLess(), ctx->stream));
+            VO_TRY(vo_reserve(ctx, ctx->d_sift_sort, tb));
+            VO_CUDA(ctx, cub::DeviceMergeSort::SortKeysCopy(ctx->d_sift_sort.p, tb, kps, sorted, n_kp, SiftKpLess(), ctx->stream));
+            // CUB's merge sort: one block-sort launch, then a partition and a merge launch per pass over the tiles
+            const int tile = cub::detail::merge_sort::policy_hub<SiftKp*>::MaxPolicy::MergeSortPolicy::ITEMS_PER_TILE;
+            int passes = 0;
+            for (int t = 1; t < (n_kp + tile - 1) / tile; t *= 2) ++passes;
+            ctx->launches += 1 + 2 * passes;
+        }
+        sift_dedup_kernel<<<nf, SIFT_DEDUP_T, 0, ctx->stream>>>(sorted, n_kp, kps, (float*)ctx->d_sift_out[0].p, base, d_n_frame + f0,
+                                                              d_first_row + f0);
+        ctx->launches++;
+        if (n_kp > 0 && want_desc) {
+            sift_descriptor_kernel<<<n_kp, SIFT_DESC_T, 0, ctx->stream>>>(P, kps, n_kp, (float*)ctx->d_sift_out[1].p + (size_t)base * 128);
+            ctx->launches++;
+        }
+        VO_CUDA(ctx, cudaGetLastError());
+        base += n_kp;
+    }
+    *n_rows = base;
+    return 0;
+}
+
+extern "C" int b200vo_sift_detect_and_compute(b200vo_ctx* ctx, const uint8_t* img, int rows, int cols, size_t step, int max_kp,
+                                              float* kps_out, float* desc_out, int32_t* n_out)
+{
+    if (!ctx || !img || !n_out || rows <= 0 || cols <= 0 || step < (size_t)cols || max_kp < 0 || (max_kp > 0 && !kps_out))
+        return B200VO_E_BADARG;
+    *n_out = 0;
+    VO_CUDA(ctx, cudaSetDevice(ctx->device));
+    VO_CUDA(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
+    // upload (tight rows)
+    VO_TRY(vo_reserve(ctx, ctx->d_stage_img[0], (size_t)rows * cols + 256));
+    uint8_t* raw = (uint8_t*)ctx->d_stage_img[0].p;
+    int* d_small = (int*)(raw + vo_align((size_t)rows * cols, 128));   // count | first row
+    VO_CUDA(ctx, cudaMemcpy2DAsync(raw, cols, img, step, cols, rows, cudaMemcpyHostToDevice, ctx->stream));
+    int n_rows = 0;
+    VO_TRY(vo_sift_frames(ctx, raw, (size_t)rows * cols, 1, rows, cols, desc_out != nullptr, d_small, d_small + 1, &n_rows));
+    // rows [0, count) of the outputs are the keypoints in cv2's order
+    const size_t b_k = vo_align((size_t)n_rows * 24, 256), b_d = desc_out ? (size_t)n_rows * 512 : 0;
+    VO_TRY(vo_reserve_pinned(ctx, 256 + b_k + b_d));
+    uint8_t* hp = (uint8_t*)ctx->h_pin;
+    VO_CUDA(ctx, cudaMemcpyAsync(hp, d_small, 4, cudaMemcpyDeviceToHost, ctx->stream));
+    if (n_rows > 0) {
+        VO_CUDA(ctx, cudaMemcpyAsync(hp + 256, ctx->d_sift_out[0].p, (size_t)n_rows * 24, cudaMemcpyDeviceToHost, ctx->stream));
+        if (desc_out) VO_CUDA(ctx, cudaMemcpyAsync(hp + 256 + b_k, ctx->d_sift_out[1].p, b_d, cudaMemcpyDeviceToHost, ctx->stream));
     }
     VO_CUDA(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
     VO_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     cudaEventElapsedTime(&ctx->last_ms, ctx->ev0, ctx->ev1);
-    // KeyPointsFilter::removeDuplicatedSorted (features2d/src/keypoint.cpp): sort, then drop equal (pt, size, angle)
-    std::vector<SiftHostKp> v((size_t)n_kp);
-    for (int i = 0; i < n_kp; ++i) v[i] = {hk[i].x, hk[i].y, hk[i].size, hk[i].angle, hk[i].response, hk[i].octave_code, i};
-    std::sort(v.begin(), v.end(), [](const SiftHostKp& a, const SiftHostKp& b) {
-        if (a.x != b.x) return a.x < b.x;
-        if (a.y != b.y) return a.y < b.y;
-        if (a.size != b.size) return a.size > b.size;
-        if (a.angle != b.angle) return a.angle < b.angle;
-        if (a.response != b.response) return a.response > b.response;
-        if (a.octave != b.octave) return a.octave > b.octave;
-        return a.src < b.src;      // full duplicates: any order (they are identical, descriptors included)
-    });
-    int cnt = 0;
-    if (n_kp > 0) {
-        int i = 0;
-        for (int j = 1; j < n_kp; ++j)
-            if (v[i].x != v[j].x || v[i].y != v[j].y || v[i].size != v[j].size || v[i].angle != v[j].angle) v[++i] = v[j];
-        cnt = i + 1;
-    }
+    const int cnt = *(const int*)hp;
     const int n_w = cnt < max_kp ? cnt : max_kp;
-    for (int i = 0; i < n_w; ++i) {
-        // firstOctave = -1: back to the input image's coordinates
-        const int oc = (v[i].octave & ~255) | ((v[i].octave - 1) & 255);
-        float* o = kps_out + (size_t)i * 6;
-        o[0] = v[i].x * 0.5f; o[1] = v[i].y * 0.5f; o[2] = v[i].size * 0.5f; o[3] = v[i].angle; o[4] = v[i].response;
-        memcpy(&o[5], &oc, 4);
-        if (desc_out) memcpy(desc_out + (size_t)i * 128, hd.data() + (size_t)v[i].src * 128, 512);
+    if (n_w > 0) {
+        memcpy(kps_out, hp + 256, (size_t)n_w * 24);
+        if (desc_out) memcpy(desc_out, hp + 256 + b_k, (size_t)n_w * 512);
     }
     *n_out = cnt;
     return 0;
