@@ -22,37 +22,17 @@ compact_tracked_kernel(int cap, const int* __restrict__ n_lm, const float* __res
                        float* __restrict__ c_obj, float* __restrict__ c_img, int* __restrict__ c_n,
                        int* __restrict__ c_orig)
 {
-    __shared__ int s_warp[8];
-    __shared__ int s_base;
     const int b = blockIdx.x;
     const int n = min(max(n_lm[b], 0), cap);   // a count beyond the slot capacity must not reach the neighbour's arrays
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    if (threadIdx.x == 0) s_base = 0;
-    __syncthreads();
-    for (int base = 0; base < n; base += blockDim.x) {
-        const int i = base + threadIdx.x;
-        const size_t gi = (size_t)b * cap + i;
-        const bool keep = i < n && lm_status[gi] == 1;
-        const unsigned bm = __ballot_sync(0xffffffffu, keep);
-        if (lane == 0) s_warp[warp] = __popc(bm);
-        __syncthreads();
-        int off = s_base;
-        for (int w = 0; w < warp; ++w) off += s_warp[w];
-        if (keep) {
-            const size_t o = (size_t)b * cap + off + __popc(bm & ((1u << lane) - 1));
-            c_obj[3 * o] = lm_obj[3 * gi]; c_obj[3 * o + 1] = lm_obj[3 * gi + 1]; c_obj[3 * o + 2] = lm_obj[3 * gi + 2];
-            c_img[2 * o] = lm_next[2 * gi]; c_img[2 * o + 1] = lm_next[2 * gi + 1];
-            c_orig[o] = i;
-        }
-        __syncthreads();
-        if (threadIdx.x == 0) {
-            int tot = 0;
-            for (int w = 0; w < 8; ++w) tot += s_warp[w];
-            s_base += tot;
-        }
-        __syncthreads();
-    }
-    if (threadIdx.x == 0) c_n[b] = s_base;
+    const size_t sb = (size_t)b * cap;
+    const int cnt = cta_compact<256>(n, [&](int i) { return lm_status[sb + i] == 1; },
+                                     [&](int i, int k) {
+                                         const size_t gi = sb + i, o = sb + k;
+                                         c_obj[3 * o] = lm_obj[3 * gi]; c_obj[3 * o + 1] = lm_obj[3 * gi + 1]; c_obj[3 * o + 2] = lm_obj[3 * gi + 2];
+                                         c_img[2 * o] = lm_next[2 * gi]; c_img[2 * o + 1] = lm_next[2 * gi + 1];
+                                         c_orig[o] = i;
+                                     });
+    if (threadIdx.x == 0) c_n[b] = cnt;
 }
 
 // inlier mask over the ORIGINAL landmark slots

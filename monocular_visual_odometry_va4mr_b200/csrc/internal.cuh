@@ -94,6 +94,39 @@ int vo_reserve_pinned(b200vo_ctx* ctx, size_t bytes);
 
 static inline size_t vo_align(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
+// Ordered compaction of [0, n) by one CTA of T threads: emit(i, o) for every i with keep(i), o = its rank among the
+// kept ones (what numpy's boolean indexing does).  keep(i) is evaluated once for every i < n.  Returns the count to
+// every thread; the trailing barrier makes back-to-back calls safe.
+template <int T, class Keep, class Emit>
+__device__ __forceinline__ int cta_compact(int n, Keep keep, Emit emit)
+{
+    __shared__ int s_warp[T / 32];
+    __shared__ int s_base;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    if (threadIdx.x == 0) s_base = 0;
+    __syncthreads();
+    for (int base = 0; base < n; base += T) {
+        const int i = base + threadIdx.x;
+        const bool k = i < n && keep(i);
+        const unsigned bm = __ballot_sync(0xffffffffu, k);
+        if (lane == 0) s_warp[warp] = __popc(bm);
+        __syncthreads();
+        int off = s_base;
+        for (int w = 0; w < warp; ++w) off += s_warp[w];
+        if (k) emit(i, off + __popc(bm & ((1u << lane) - 1)));
+        __syncthreads();
+        if (threadIdx.x == 0) {
+            int tot = 0;
+            for (int w = 0; w < T / 32; ++w) tot += s_warp[w];
+            s_base += tot;
+        }
+        __syncthreads();
+    }
+    const int r = s_base;
+    __syncthreads();
+    return r;
+}
+
 // ---- pyramid.cu ----
 int vo_pyr_levels(int w, int h, int win_w, int win_h, int max_level);
 void vo_pyr_geom(int rows, int cols, int levels, PyrGeom* g);

@@ -14,28 +14,6 @@
 
 using namespace vo;
 
-// ---- f2: one warp per new corner, lanes stride over the existing candidates ----
-__global__ void __launch_bounds__(256)
-min_distance_kernel(const float2* __restrict__ pts, int n, const float2* __restrict__ existing, int m, float min_dist,
-                    uint8_t* __restrict__ valid)
-{
-    const int i = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
-    if (i >= n) return;
-    const float2 p = pts[i];
-    bool ok = true;
-    for (int j0 = 0; j0 < m; j0 += 32) {
-        const int j = j0 + lane;
-        if (j < m) {
-            const float2 q = existing[j];
-            const float dx = __fsub_rn(p.x, q.x), dy = __fsub_rn(p.y, q.y);
-            const float d = __fsqrt_rn(__fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy)));
-            ok = d > min_dist;           // NaN compares false, as in numpy
-        }
-        if (!__all_sync(0xffffffffu, ok)) { ok = false; break; }
-    }
-    if (lane == 0) valid[i] = ok ? 1 : 0;
-}
-
 __device__ __forceinline__ void invert_pose(const double* cw, double* R, double* t)
 {
 #pragma unroll
@@ -107,50 +85,8 @@ __device__ __forceinline__ void triangulate_one(const TriArgs& a, int i)
     }
 }
 
-__global__ void __launch_bounds__(64)
-triangulate_kernel(TriArgs a)
-{
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < a.n) triangulate_one(a, i);
-}
-
-// ordered compaction of the accepted candidates (keep == 0): one CTA, ballot + running base
-__device__ __forceinline__ void triangulate_compact_block(const TriArgs& a)
-{
-    __shared__ int s_warp[32];
-    __shared__ int s_base;
-    if (threadIdx.x == 0) s_base = 0;
-    __syncthreads();
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    for (int base = 0; base < a.n; base += blockDim.x) {
-        const int i = base + threadIdx.x;
-        const bool acc = i < a.n && a.keep[i] == 0;
-        const unsigned bm = __ballot_sync(0xffffffffu, acc);
-        if (lane == 0) s_warp[warp] = __popc(bm);
-        __syncthreads();
-        int off = s_base;
-        for (int w = 0; w < warp; ++w) off += s_warp[w];
-        if (acc) {
-            const int o = off + __popc(bm & ((1u << lane) - 1));
-            a.out_lm[3 * o] = a.lm_slot[3 * i]; a.out_lm[3 * o + 1] = a.lm_slot[3 * i + 1]; a.out_lm[3 * o + 2] = a.lm_slot[3 * i + 2];
-            a.out_kp[2 * o] = a.keys[2 * i]; a.out_kp[2 * o + 1] = a.keys[2 * i + 1];
-        }
-        __syncthreads();
-        if (threadIdx.x == 0) {
-            int tot = 0;
-            for (int w = 0; w < 32; ++w) tot += s_warp[w];
-            s_base += tot;
-        }
-        __syncthreads();
-    }
-    if (threadIdx.x == 0) *a.n_new = s_base;
-}
-
-__global__ void __launch_bounds__(1024)
-triangulate_compact_kernel(TriArgs a) { triangulate_compact_block(a); }
-
-// ---- batched forms (SURVEY 8f "batched f1/f2 on the resident batch state"): the same per-sequence work for every
-// sequence of a batch in one launch each; blockIdx.y = sequence, ragged counts per sequence ----
+// ---- f1 and f2 for a batch of sequences (SURVEY 8f "batched f1/f2 on the resident batch state") in one launch each;
+// blockIdx.y = sequence, ragged counts per sequence.  The per-sequence entry points are the batch of one ----
 __device__ __forceinline__ TriArgs tri_sequence(const TriBatchArgs& b, int s)
 {
     TriArgs a = b.common;
@@ -174,13 +110,19 @@ triangulate_batch_kernel(TriBatchArgs b)
     if (i < a.n) triangulate_one(a, i);
 }
 
+// ordered compaction of the accepted candidates (keep == 0): one CTA per sequence
 __global__ void __launch_bounds__(1024)
 triangulate_compact_batch_kernel(TriBatchArgs b)
 {
     const TriArgs a = tri_sequence(b, blockIdx.x);
-    triangulate_compact_block(a);
+    const int cnt = cta_compact<1024>(a.n, [&](int i) { return a.keep[i] == 0; }, [&](int i, int o) {
+        a.out_lm[3 * o] = a.lm_slot[3 * i]; a.out_lm[3 * o + 1] = a.lm_slot[3 * i + 1]; a.out_lm[3 * o + 2] = a.lm_slot[3 * i + 2];
+        a.out_kp[2 * o] = a.keys[2 * i]; a.out_kp[2 * o + 1] = a.keys[2 * i + 1];
+    });
+    if (threadIdx.x == 0) *a.n_new = cnt;
 }
 
+// f2: one warp per new corner, lanes stride over the existing candidates
 __global__ void __launch_bounds__(256)
 min_distance_batch_kernel(const float2* __restrict__ pts, const int* __restrict__ n, int n_cap, const float2* __restrict__ existing,
                           const int* __restrict__ m, int m_cap, float min_dist, uint8_t* __restrict__ valid)
@@ -233,99 +175,11 @@ int vo_min_distance_batch_launch(b200vo_ctx* ctx, int batch, const float* pts, c
     return 0;
 }
 
-extern "C" int b200vo_min_distance_mask(b200vo_ctx* ctx, const float* pts, int n, const float* existing, int m,
-                                        float min_dist, uint8_t* valid)
+// Body of both f2 entry points: stages pts (batch, n_cap, 2), existing (batch, m_cap, 2) and the counts in the pinned
+// block, runs the kernel and waits.  *valid_h points at the result in the pinned block: uint8 (batch, n_cap), rows >= n[s] 0.
+static int min_distance_staged(b200vo_ctx* ctx, int batch, const float* pts, const int32_t* n, int n_cap, const float* existing,
+                               const int32_t* m, int m_cap, float min_dist, const uint8_t** valid_h)
 {
-    if (!ctx || n < 0 || m < 0 || (n > 0 && (!pts || !valid)) || (m > 0 && !existing)) return B200VO_E_BADARG;
-    if (n == 0) return 0;
-    VO_CUDA(ctx, cudaSetDevice(ctx->device));
-    VO_CUDA(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
-    const size_t b_p = vo_align((size_t)n * 8, 256), b_e = vo_align((size_t)(m > 0 ? m : 1) * 8, 256), b_v = vo_align((size_t)n, 256);
-    VO_TRY(vo_reserve(ctx, ctx->d_scratch[6], b_p + b_e + b_v));
-    VO_TRY(vo_reserve_pinned(ctx, b_p + b_e + b_v));
-    uint8_t* d = (uint8_t*)ctx->d_scratch[6].p;
-    uint8_t* hp = (uint8_t*)ctx->h_pin;
-    memcpy(hp, pts, (size_t)n * 8);
-    if (m > 0) memcpy(hp + b_p, existing, (size_t)m * 8);
-    VO_CUDA(ctx, cudaMemcpyAsync(d, hp, b_p + b_e, cudaMemcpyHostToDevice, ctx->stream));
-    min_distance_kernel<<<(n * 32 + 255) / 256, 256, 0, ctx->stream>>>((const float2*)d, n, (const float2*)(d + b_p), m, min_dist,
-                                                                      d + b_p + b_e);
-    ctx->launches++;
-    VO_CUDA(ctx, cudaGetLastError());
-    VO_CUDA(ctx, cudaMemcpyAsync(hp + b_p + b_e, d + b_p + b_e, (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
-    VO_CUDA(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
-    VO_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    cudaEventElapsedTime(&ctx->last_ms, ctx->ev0, ctx->ev1);
-    memcpy(valid, hp + b_p + b_e, (size_t)n);
-    return 0;
-}
-
-extern "C" int b200vo_triangulate_landmarks(b200vo_ctx* ctx, const double K[9], double min_dist, double max_dist,
-                                            double min_baseline_angle_deg, int min_baseline_frames,
-                                            const float* first_keys, const float* keys, const int32_t* first_pose, int n,
-                                            const double* poses_cw, int n_poses, const double cur_pose_cw[12],
-                                            uint8_t* too_short_baseline, float* new_landmarks, float* new_keypoints,
-                                            int* n_new)
-{
-    if (!ctx || !K || !cur_pose_cw || !n_new || n < 0 || n_poses < 1 || !poses_cw) return B200VO_E_BADARG;
-    *n_new = 0;
-    if (n == 0) return 0;
-    if (!first_keys || !keys || !first_pose || !too_short_baseline || !new_landmarks || !new_keypoints)
-        return vo_set_err(ctx, B200VO_E_BADARG, "null pointer");
-    VO_CUDA(ctx, cudaSetDevice(ctx->device));
-    VO_CUDA(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
-    TriArgs a{};
-    for (int k = 0; k < 9; ++k) a.K[k] = K[k];
-    const double Ki[9] = {1.0 / K[0], 0, -K[2] / K[0], 0, 1.0 / K[4], -K[5] / K[4], 0, 0, 1};
-    for (int k = 0; k < 9; ++k) a.Ki[k] = Ki[k];
-    for (int k = 0; k < 12; ++k) a.cur[k] = cur_pose_cw[k];
-    a.min_dist = min_dist; a.max_dist = max_dist; a.min_angle_deg = min_baseline_angle_deg;
-    a.min_frames = min_baseline_frames; a.n = n; a.n_poses = n_poses;
-    // device layout: inputs [first_keys | keys | first_pose | poses] then outputs [keep | out_lm | out_kp | n_new,flags] + lm_slot
-    const size_t b_k = vo_align((size_t)n * 8, 256), b_fp = vo_align((size_t)n * 4, 256), b_ps = vo_align((size_t)n_poses * 96, 256);
-    const size_t b_keep = vo_align((size_t)n, 256), b_lm = vo_align((size_t)n * 12, 256), b_small = 256;
-    const size_t in_bytes = 2 * b_k + b_fp + b_ps, out_bytes = b_keep + b_lm + b_k + b_small;
-    VO_TRY(vo_reserve(ctx, ctx->d_scratch[7], in_bytes + out_bytes + b_lm));
-    VO_TRY(vo_reserve_pinned(ctx, in_bytes + out_bytes));
-    uint8_t* d = (uint8_t*)ctx->d_scratch[7].p;
-    uint8_t* hp = (uint8_t*)ctx->h_pin;
-    memcpy(hp, first_keys, (size_t)n * 8);
-    memcpy(hp + b_k, keys, (size_t)n * 8);
-    memcpy(hp + 2 * b_k, first_pose, (size_t)n * 4);
-    memcpy(hp + 2 * b_k + b_fp, poses_cw, (size_t)n_poses * 96);
-    VO_CUDA(ctx, cudaMemcpyAsync(d, hp, in_bytes, cudaMemcpyHostToDevice, ctx->stream));
-    a.first_keys = (const float*)d; a.keys = (const float*)(d + b_k); a.first_pose = (const int*)(d + 2 * b_k);
-    a.poses = (const double*)(d + 2 * b_k + b_fp);
-    uint8_t* dout = d + in_bytes;
-    a.keep = dout; a.out_lm = (float*)(dout + b_keep); a.out_kp = (float*)(dout + b_keep + b_lm);
-    a.n_new = (int*)(dout + b_keep + b_lm + b_k); a.flags = a.n_new + 1;
-    a.lm_slot = (float*)(dout + out_bytes);
-    VO_CUDA(ctx, cudaMemsetAsync(a.n_new, 0, b_small, ctx->stream));
-    triangulate_kernel<<<(n + 63) / 64, 64, 0, ctx->stream>>>(a);
-    triangulate_compact_kernel<<<1, 1024, 0, ctx->stream>>>(a);
-    ctx->launches += 2;
-    VO_CUDA(ctx, cudaGetLastError());
-    uint8_t* ho = hp + in_bytes;
-    VO_CUDA(ctx, cudaMemcpyAsync(ho, dout, out_bytes, cudaMemcpyDeviceToHost, ctx->stream));
-    VO_CUDA(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
-    VO_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    cudaEventElapsedTime(&ctx->last_ms, ctx->ev0, ctx->ev1);
-    const int* small = (const int*)(ho + b_keep + b_lm + b_k);
-    if (small[1] & 1) return vo_set_err(ctx, B200VO_E_BADARG, "first_pose index outside [0, n_poses)");
-    const int cnt = small[0];
-    memcpy(too_short_baseline, ho, (size_t)n);
-    memcpy(new_landmarks, ho + b_keep, (size_t)cnt * 12);
-    memcpy(new_keypoints, ho + b_keep + b_lm, (size_t)cnt * 8);
-    *n_new = cnt;
-    return 0;
-}
-
-// Batched f2: the candidate min-distance filter (:258) for every sequence of a batch in one launch.
-// pts float32 (batch, n_cap, 2) with n[batch] live rows, existing float32 (batch, m_cap, 2) with m[batch]; valid uint8 (batch, n_cap).
-extern "C" int b200vo_batch_min_distance_mask(b200vo_ctx* ctx, int batch, const float* pts, const int32_t* n, int n_cap,
-                                              const float* existing, const int32_t* m, int m_cap, float min_dist, uint8_t* valid)
-{
-    if (!ctx || batch < 1 || n_cap < 1 || m_cap < 0 || !pts || !n || !m || !valid || (m_cap > 0 && !existing)) return B200VO_E_BADARG;
     VO_CUDA(ctx, cudaSetDevice(ctx->device));
     VO_CUDA(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
     const int mc = m_cap > 0 ? m_cap : 1;
@@ -341,7 +195,9 @@ extern "C" int b200vo_batch_min_distance_mask(b200vo_ctx* ctx, int batch, const 
     memcpy(hp + b_p + b_e + b_c, m, (size_t)batch * 4);
     VO_CUDA(ctx, cudaMemcpyAsync(d, hp, b_p + b_e + 2 * b_c, cudaMemcpyHostToDevice, ctx->stream));
     uint8_t* dv = d + b_p + b_e + 2 * b_c;
-    VO_CUDA(ctx, cudaMemsetAsync(dv, 0, b_v, ctx->stream));
+    bool full = true;   // every row is live (the batch of one): the kernel writes all of them, nothing to clear
+    for (int s = 0; s < batch; ++s) full = full && n[s] >= n_cap;
+    if (!full) VO_CUDA(ctx, cudaMemsetAsync(dv, 0, b_v, ctx->stream));
     VO_TRY(vo_min_distance_batch_launch(ctx, batch, (const float*)d, (const int*)(d + b_p + b_e), n_cap, (const float*)(d + b_p),
                                         (const int*)(d + b_p + b_e + b_c), m_cap, min_dist, dv, ctx->stream));
     uint8_t* ho = hp + b_p + b_e + 2 * b_c;
@@ -349,24 +205,25 @@ extern "C" int b200vo_batch_min_distance_mask(b200vo_ctx* ctx, int batch, const 
     VO_CUDA(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
     VO_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     cudaEventElapsedTime(&ctx->last_ms, ctx->ev0, ctx->ev1);
-    memcpy(valid, ho, (size_t)batch * n_cap);
+    *valid_h = ho;
     return 0;
 }
 
-// Batched f1: the candidate loop of triangulate_landmarks (:170-204) for every sequence of a batch: two launches.
-// Per sequence s: n[s] candidates in rows [0, n[s]) of the (batch, cap, ...) arrays, n_poses[s] stored poses in
-// poses_cw (batch, pose_cap, 12), the current pose cur_pose_cw (batch, 12).  Outputs: too_short_baseline uint8 (batch, cap),
-// new_landmarks float32 (batch, cap, 3) / new_keypoints float32 (batch, cap, 2) compacted per sequence, n_new int32 (batch).
-extern "C" int b200vo_batch_triangulate_landmarks(b200vo_ctx* ctx, const double K[9], double min_dist, double max_dist,
-                                                  double min_baseline_angle_deg, int min_baseline_frames, int batch, int cap,
-                                                  const float* first_keys, const float* keys, const int32_t* first_pose,
-                                                  const int32_t* n, const double* poses_cw, const int32_t* n_poses, int pose_cap,
-                                                  const double* cur_pose_cw, uint8_t* too_short_baseline, float* new_landmarks,
-                                                  float* new_keypoints, int32_t* n_new)
+// The results of triangulate_staged in the pinned block, laid out as the batched entry point returns them
+struct TriResults {
+    const uint8_t* keep;       // [batch][cap] too_short_baseline
+    const float* lm;           // [batch][cap][3] compacted per sequence
+    const float* kp;           // [batch][cap][2]
+    const int* n_new;          // [batch]
+    const int* flags;          // [batch] bit0: first_pose out of range
+};
+
+// Body of both f1 entry points: stages the (batch, cap, ...) inputs in the pinned block, runs the two kernels and waits.
+static int triangulate_staged(b200vo_ctx* ctx, const double K[9], double min_dist, double max_dist, double min_baseline_angle_deg,
+                              int min_baseline_frames, int batch, int cap, const float* first_keys, const float* keys,
+                              const int32_t* first_pose, const int32_t* n, const double* poses_cw, const int32_t* n_poses, int pose_cap,
+                              const double* cur_pose_cw, TriResults* res)
 {
-    if (!ctx || !K || batch < 1 || cap < 1 || pose_cap < 1 || !first_keys || !keys || !first_pose || !n || !poses_cw || !n_poses ||
-        !cur_pose_cw || !too_short_baseline || !new_landmarks || !new_keypoints || !n_new)
-        return B200VO_E_BADARG;
     VO_CUDA(ctx, cudaSetDevice(ctx->device));
     VO_CUDA(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
     TriBatchArgs b{};
@@ -401,13 +258,82 @@ extern "C" int b200vo_batch_triangulate_landmarks(b200vo_ctx* ctx, const double 
     VO_CUDA(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
     VO_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     cudaEventElapsedTime(&ctx->last_ms, ctx->ev0, ctx->ev1);
-    const int* flg = (const int*)(ho + b_keep + b_lm + b_k + b_cnt);
+    res->keep = ho; res->lm = (const float*)(ho + b_keep); res->kp = (const float*)(ho + b_keep + b_lm);
+    res->n_new = (const int*)(ho + b_keep + b_lm + b_k); res->flags = (const int*)(ho + b_keep + b_lm + b_k + b_cnt);
+    return 0;
+}
+
+extern "C" int b200vo_min_distance_mask(b200vo_ctx* ctx, const float* pts, int n, const float* existing, int m,
+                                        float min_dist, uint8_t* valid)
+{
+    if (!ctx || n < 0 || m < 0 || (n > 0 && (!pts || !valid)) || (m > 0 && !existing)) return B200VO_E_BADARG;
+    if (n == 0) return 0;
+    const uint8_t* h;
+    VO_TRY(min_distance_staged(ctx, 1, pts, &n, n, existing, &m, m, min_dist, &h));
+    memcpy(valid, h, (size_t)n);
+    return 0;
+}
+
+extern "C" int b200vo_triangulate_landmarks(b200vo_ctx* ctx, const double K[9], double min_dist, double max_dist,
+                                            double min_baseline_angle_deg, int min_baseline_frames,
+                                            const float* first_keys, const float* keys, const int32_t* first_pose, int n,
+                                            const double* poses_cw, int n_poses, const double cur_pose_cw[12],
+                                            uint8_t* too_short_baseline, float* new_landmarks, float* new_keypoints,
+                                            int* n_new)
+{
+    if (!ctx || !K || !cur_pose_cw || !n_new || n < 0 || n_poses < 1 || !poses_cw) return B200VO_E_BADARG;
+    *n_new = 0;
+    if (n == 0) return 0;
+    if (!first_keys || !keys || !first_pose || !too_short_baseline || !new_landmarks || !new_keypoints)
+        return vo_set_err(ctx, B200VO_E_BADARG, "null pointer");
+    TriResults r;
+    VO_TRY(triangulate_staged(ctx, K, min_dist, max_dist, min_baseline_angle_deg, min_baseline_frames, 1, n, first_keys, keys,
+                              first_pose, &n, poses_cw, &n_poses, n_poses, cur_pose_cw, &r));
+    if (r.flags[0] & 1) return vo_set_err(ctx, B200VO_E_BADARG, "first_pose index outside [0, n_poses)");
+    const int cnt = r.n_new[0];
+    memcpy(too_short_baseline, r.keep, (size_t)n);
+    memcpy(new_landmarks, r.lm, (size_t)cnt * 12);
+    memcpy(new_keypoints, r.kp, (size_t)cnt * 8);
+    *n_new = cnt;
+    return 0;
+}
+
+// Batched f2: the candidate min-distance filter (:258) for every sequence of a batch in one launch.
+// pts float32 (batch, n_cap, 2) with n[batch] live rows, existing float32 (batch, m_cap, 2) with m[batch]; valid uint8 (batch, n_cap).
+extern "C" int b200vo_batch_min_distance_mask(b200vo_ctx* ctx, int batch, const float* pts, const int32_t* n, int n_cap,
+                                              const float* existing, const int32_t* m, int m_cap, float min_dist, uint8_t* valid)
+{
+    if (!ctx || batch < 1 || n_cap < 1 || m_cap < 0 || !pts || !n || !m || !valid || (m_cap > 0 && !existing)) return B200VO_E_BADARG;
+    const uint8_t* h;
+    VO_TRY(min_distance_staged(ctx, batch, pts, n, n_cap, existing, m, m_cap, min_dist, &h));
+    memcpy(valid, h, (size_t)batch * n_cap);
+    return 0;
+}
+
+// Batched f1: the candidate loop of triangulate_landmarks (:170-204) for every sequence of a batch: two launches.
+// Per sequence s: n[s] candidates in rows [0, n[s]) of the (batch, cap, ...) arrays, n_poses[s] stored poses in
+// poses_cw (batch, pose_cap, 12), the current pose cur_pose_cw (batch, 12).  Outputs: too_short_baseline uint8 (batch, cap),
+// new_landmarks float32 (batch, cap, 3) / new_keypoints float32 (batch, cap, 2) compacted per sequence, n_new int32 (batch).
+extern "C" int b200vo_batch_triangulate_landmarks(b200vo_ctx* ctx, const double K[9], double min_dist, double max_dist,
+                                                  double min_baseline_angle_deg, int min_baseline_frames, int batch, int cap,
+                                                  const float* first_keys, const float* keys, const int32_t* first_pose,
+                                                  const int32_t* n, const double* poses_cw, const int32_t* n_poses, int pose_cap,
+                                                  const double* cur_pose_cw, uint8_t* too_short_baseline, float* new_landmarks,
+                                                  float* new_keypoints, int32_t* n_new)
+{
+    if (!ctx || !K || batch < 1 || cap < 1 || pose_cap < 1 || !first_keys || !keys || !first_pose || !n || !poses_cw || !n_poses ||
+        !cur_pose_cw || !too_short_baseline || !new_landmarks || !new_keypoints || !n_new)
+        return B200VO_E_BADARG;
+    TriResults r;
+    VO_TRY(triangulate_staged(ctx, K, min_dist, max_dist, min_baseline_angle_deg, min_baseline_frames, batch, cap, first_keys, keys,
+                              first_pose, n, poses_cw, n_poses, pose_cap, cur_pose_cw, &r));
     for (int s = 0; s < batch; ++s)
-        if (flg[s] & 1) return vo_set_err(ctx, B200VO_E_BADARG, "sequence %d: first_pose index outside [0, n_poses)", s);
-    memcpy(too_short_baseline, ho, nc);
-    memcpy(new_landmarks, ho + b_keep, nc * 12);
-    memcpy(new_keypoints, ho + b_keep + b_lm, nc * 8);
-    memcpy(n_new, ho + b_keep + b_lm + b_k, (size_t)batch * 4);
+        if (r.flags[s] & 1) return vo_set_err(ctx, B200VO_E_BADARG, "sequence %d: first_pose index outside [0, n_poses)", s);
+    const size_t nc = (size_t)batch * cap;
+    memcpy(too_short_baseline, r.keep, nc);
+    memcpy(new_landmarks, r.lm, nc * 12);
+    memcpy(new_keypoints, r.kp, nc * 8);
+    memcpy(n_new, r.n_new, (size_t)batch * 4);
     return 0;
 }
 

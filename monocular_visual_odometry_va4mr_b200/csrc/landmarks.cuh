@@ -3,6 +3,7 @@
 #pragma once
 #include "internal.cuh"
 
+// one sequence's view of the triangulation kernels, built on the device by tri_sequence
 struct TriArgs {
     double K[9], Ki[9];
     double cur[12];            // R_CW | t_CW of the current frame (as the reference stores them)

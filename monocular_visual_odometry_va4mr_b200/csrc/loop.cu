@@ -48,38 +48,6 @@ struct LoopDev {   // kernel view of the state and of the step's scratch (device
     int* n_corner; uint8_t* valid;             // corners per sequence, distance-filter result [batch][G]
 };
 
-// Ordered compaction of [0, n) by one CTA of LOOP_T threads: emit(i, o) for every i with keep(i), o = its rank among
-// the kept ones (what numpy's boolean indexing does).  Returns the count to every thread.
-template <class Keep, class Emit>
-__device__ __forceinline__ int cta_compact(int n, Keep keep, Emit emit)
-{
-    __shared__ int s_warp[LOOP_T / 32];
-    __shared__ int s_base;
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    if (threadIdx.x == 0) s_base = 0;
-    __syncthreads();
-    for (int base = 0; base < n; base += LOOP_T) {
-        const int i = base + threadIdx.x;
-        const bool k = i < n && keep(i);
-        const unsigned bm = __ballot_sync(0xffffffffu, k);
-        if (lane == 0) s_warp[warp] = __popc(bm);
-        __syncthreads();
-        int off = s_base;
-        for (int w = 0; w < warp; ++w) off += s_warp[w];
-        if (k) emit(i, off + __popc(bm & ((1u << lane) - 1)));
-        __syncthreads();
-        if (threadIdx.x == 0) {
-            int tot = 0;
-            for (int w = 0; w < LOOP_T / 32; ++w) tot += s_warp[w];
-            s_base += tot;
-        }
-        __syncthreads();
-    }
-    const int r = s_base;
-    __syncthreads();
-    return r;
-}
-
 // Steps 3-5 of MiniVO.step and the status filter of step 2: one CTA per sequence.
 __global__ void __launch_bounds__(LOOP_T)
 loop_commit_kernel(LoopDev d, LoopOut out)
@@ -124,12 +92,12 @@ loop_commit_kernel(LoopDev d, LoopOut out)
     const size_t co = (size_t)s * d.C;
     const bool tracked = d.trk_cand[s] > 0;
     const float* kin = tracked ? d.cand_next : d.keys;
-    const int nc = cta_compact(d.n_cand[s], [&](int i) { return !tracked || d.cand_status[co + i] == 1; },
-                               [&](int i, int o) {
-                                   d.keys_b[2 * (co + o)] = kin[2 * (co + i)]; d.keys_b[2 * (co + o) + 1] = kin[2 * (co + i) + 1];
-                                   d.fkeys_b[2 * (co + o)] = d.fkeys[2 * (co + i)]; d.fkeys_b[2 * (co + o) + 1] = d.fkeys[2 * (co + i) + 1];
-                                   d.fpose_b[co + o] = d.fpose[co + i];
-                               });
+    const int nc = cta_compact<LOOP_T>(d.n_cand[s], [&](int i) { return !tracked || d.cand_status[co + i] == 1; },
+                                       [&](int i, int o) {
+                                           d.keys_b[2 * (co + o)] = kin[2 * (co + i)]; d.keys_b[2 * (co + o) + 1] = kin[2 * (co + i) + 1];
+                                           d.fkeys_b[2 * (co + o)] = d.fkeys[2 * (co + i)]; d.fkeys_b[2 * (co + o) + 1] = d.fkeys[2 * (co + i) + 1];
+                                           d.fpose_b[co + o] = d.fpose[co + i];
+                                       });
     if (tid == 0) {
         d.n_lm[s] = m;
         d.n_cand_b[s] = nc;
@@ -153,12 +121,12 @@ loop_merge_kernel(LoopDev d)
             d.lm[3 * o] = d.new_lm[3 * (co + k)]; d.lm[3 * o + 1] = d.new_lm[3 * (co + k) + 1]; d.lm[3 * o + 2] = d.new_lm[3 * (co + k) + 2];
             d.lm_kp[2 * o] = d.new_kp[2 * (co + k)]; d.lm_kp[2 * o + 1] = d.new_kp[2 * (co + k) + 1];
         }
-    const int nc = cta_compact(d.n_cand_b[s], [&](int i) { return !ran || d.keep[co + i] != 0; },
-                               [&](int i, int o) {
-                                   d.keys[2 * (co + o)] = d.keys_b[2 * (co + i)]; d.keys[2 * (co + o) + 1] = d.keys_b[2 * (co + i) + 1];
-                                   d.fkeys[2 * (co + o)] = d.fkeys_b[2 * (co + i)]; d.fkeys[2 * (co + o) + 1] = d.fkeys_b[2 * (co + i) + 1];
-                                   d.fpose[co + o] = d.fpose_b[co + i];
-                               });
+    const int nc = cta_compact<LOOP_T>(d.n_cand_b[s], [&](int i) { return !ran || d.keep[co + i] != 0; },
+                                       [&](int i, int o) {
+                                           d.keys[2 * (co + o)] = d.keys_b[2 * (co + i)]; d.keys[2 * (co + o) + 1] = d.keys_b[2 * (co + i) + 1];
+                                           d.fkeys[2 * (co + o)] = d.fkeys_b[2 * (co + i)]; d.fkeys[2 * (co + o) + 1] = d.fkeys_b[2 * (co + i) + 1];
+                                           d.fpose[co + o] = d.fpose_b[co + i];
+                                       });
     if (tid == 0) {
         if (fits) d.n_lm[s] = nl + nn;
         else d.status[s] = B200VO_LOOP_OVERFLOW;
@@ -178,15 +146,15 @@ loop_append_kernel(LoopDev d, LoopOut out)
     if (s_st == B200VO_LOOP_OK) {
         const int nc = d.n_cand[s], np = d.n_poses[s];
         const size_t co = (size_t)s * d.C, go = (size_t)s * d.G;
-        const int cnt = cta_compact(d.n_corner[s], [&](int i) { return d.valid[go + i] != 0; },
-                                    [&](int i, int o) {
-                                        if (nc + o >= d.C) return;
-                                        const size_t q = co + nc + o;
-                                        const float x = d.corners[2 * (go + i)], y = d.corners[2 * (go + i) + 1];
-                                        d.keys[2 * q] = x; d.keys[2 * q + 1] = y;
-                                        d.fkeys[2 * q] = x; d.fkeys[2 * q + 1] = y;
-                                        d.fpose[q] = np;
-                                    });
+        const int cnt = cta_compact<LOOP_T>(d.n_corner[s], [&](int i) { return d.valid[go + i] != 0; },
+                                            [&](int i, int o) {
+                                                if (nc + o >= d.C) return;
+                                                const size_t q = co + nc + o;
+                                                const float x = d.corners[2 * (go + i)], y = d.corners[2 * (go + i) + 1];
+                                                d.keys[2 * q] = x; d.keys[2 * q + 1] = y;
+                                                d.fkeys[2 * q] = x; d.fkeys[2 * q + 1] = y;
+                                                d.fpose[q] = np;
+                                            });
         if (tid == 0) {
             if (nc + cnt > d.C) { d.status[s] = B200VO_LOOP_OVERFLOW; s_st = B200VO_LOOP_OVERFLOW; }
             else { d.n_cand[s] = nc + cnt; d.n_poses[s] = np + 1; }
@@ -495,12 +463,12 @@ boot_match_kernel(BootDev b)
     const float* k0 = b.kp6 + (size_t)t[BT_ROW0] * 6;
     const float* k1 = b.kp6 + (size_t)t[BT_ROW1] * 6;
     const size_t po = (size_t)k * b.cap;
-    const int n = cta_compact(nq, [&](int i) { return b.accept[qo + i] != 0; },
-                              [&](int i, int o) {
-                                  const int j = b.idx2[2 * (qo + i)];
-                                  b.pts0[2 * (po + o)] = k0[6 * i]; b.pts0[2 * (po + o) + 1] = k0[6 * i + 1];
-                                  b.pts1[2 * (po + o)] = k1[6 * j]; b.pts1[2 * (po + o) + 1] = k1[6 * j + 1];
-                              });
+    const int n = cta_compact<LOOP_T>(nq, [&](int i) { return b.accept[qo + i] != 0; },
+                                      [&](int i, int o) {
+                                          const int j = b.idx2[2 * (qo + i)];
+                                          b.pts0[2 * (po + o)] = k0[6 * i]; b.pts0[2 * (po + o) + 1] = k0[6 * i + 1];
+                                          b.pts1[2 * (po + o)] = k1[6 * j]; b.pts1[2 * (po + o) + 1] = k1[6 * j + 1];
+                                      });
     if (threadIdx.x == 0) b.n_match[k] = n;
 }
 
@@ -510,11 +478,11 @@ boot_inliers_kernel(BootDev b)
     const int k = blockIdx.x;
     const bool found = boot_found(b, k);
     const size_t po = (size_t)k * b.cap;
-    const int n = cta_compact(found ? b.n_match[k] : 0, [&](int i) { return b.emask[po + i] == 1; },
-                              [&](int i, int o) {
-                                  b.inl0[2 * (po + o)] = b.pts0[2 * (po + i)]; b.inl0[2 * (po + o) + 1] = b.pts0[2 * (po + i) + 1];
-                                  b.inl1[2 * (po + o)] = b.pts1[2 * (po + i)]; b.inl1[2 * (po + o) + 1] = b.pts1[2 * (po + i) + 1];
-                              });
+    const int n = cta_compact<LOOP_T>(found ? b.n_match[k] : 0, [&](int i) { return b.emask[po + i] == 1; },
+                                      [&](int i, int o) {
+                                          b.inl0[2 * (po + o)] = b.pts0[2 * (po + i)]; b.inl0[2 * (po + o) + 1] = b.pts0[2 * (po + i) + 1];
+                                          b.inl1[2 * (po + o)] = b.pts1[2 * (po + i)]; b.inl1[2 * (po + o) + 1] = b.pts1[2 * (po + i) + 1];
+                                      });
     if (threadIdx.x == 0) b.n_inl[k] = n;
 }
 
@@ -542,7 +510,7 @@ boot_load_kernel(LoopDev d, BootDev b)
     const bool found = boot_found(b, k);
     const int n_inl = b.n_inl[k], nn = found ? b.n_new[k] : 0;
     // the too_short_baseline candidates (keep == 1), counted before anything is written
-    const int nc = cta_compact(found ? n_inl : 0, [&](int i) { return b.keep[po + i] != 0; }, [](int, int) {});
+    const int nc = cta_compact<LOOP_T>(found ? n_inl : 0, [&](int i) { return b.keep[po + i] != 0; }, [](int, int) {});
     if (tid == 0) {
         s_code = !found ? B200VO_LOOP_NO_BOOTSTRAP : (nn > d.L || nc > d.C) ? B200VO_LOOP_OVERFLOW : B200VO_LOOP_OK;
         b.res[k] = s_code;
@@ -561,12 +529,12 @@ boot_load_kernel(LoopDev d, BootDev b)
         d.lm[3 * (lo + i) + 2] = b.new_lm[3 * (po + i) + 2];
         d.lm_kp[2 * (lo + i)] = b.new_kp[2 * (po + i)]; d.lm_kp[2 * (lo + i) + 1] = b.new_kp[2 * (po + i) + 1];
     }
-    cta_compact(n_inl, [&](int i) { return b.keep[po + i] != 0; },
-                [&](int i, int o) {
-                    d.keys[2 * (co + o)] = b.inl1[2 * (po + i)]; d.keys[2 * (co + o) + 1] = b.inl1[2 * (po + i) + 1];
-                    d.fkeys[2 * (co + o)] = b.inl0[2 * (po + i)]; d.fkeys[2 * (co + o) + 1] = b.inl0[2 * (po + i) + 1];
-                    d.fpose[co + o] = 0;
-                });
+    cta_compact<LOOP_T>(n_inl, [&](int i) { return b.keep[po + i] != 0; },
+                        [&](int i, int o) {
+                            d.keys[2 * (co + o)] = b.inl1[2 * (po + i)]; d.keys[2 * (co + o) + 1] = b.inl1[2 * (po + i) + 1];
+                            d.fkeys[2 * (co + o)] = b.inl0[2 * (po + i)]; d.fkeys[2 * (co + o) + 1] = b.inl0[2 * (po + i) + 1];
+                            d.fpose[co + o] = 0;
+                        });
     double* ph = d.poses + (size_t)s * d.P * 12;   // [I | 0], [R | t]
     if (tid < 12) ph[tid] = (tid == 0 || tid == 4 || tid == 8) ? 1.0 : 0.0;
     else if (tid < 24) ph[tid] = b.cur[12 * k + tid - 12];

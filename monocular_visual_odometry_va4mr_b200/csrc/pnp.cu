@@ -171,8 +171,6 @@ pnp_select_kernel(PnpArgs a)
 {
     __shared__ int s_win, s_run;
     __shared__ double s_h[12];
-    __shared__ int s_warp[8];
-    __shared__ int s_base;
     const int b = blockIdx.x;
     const int N = a.n[b];
     const size_t hb = (size_t)b * a.iters;
@@ -191,7 +189,7 @@ pnp_select_kernel(PnpArgs a)
             }
             run = it;
         }
-        s_win = win; s_run = run; s_base = 0;
+        s_win = win; s_run = run;
     }
     __syncthreads();
     const int win = s_win;
@@ -205,9 +203,8 @@ pnp_select_kernel(PnpArgs a)
     }
     if (threadIdx.x < 12) s_h[threadIdx.x] = a.hyp[(hb + win) * 12 + threadIdx.x];
     __syncthreads();
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    for (int base = 0; base < a.cap; base += blockDim.x) {
-        const int i = base + threadIdx.x;
+    // over every slot, so that keep() writes the whole mask
+    const int M = cta_compact<256>(a.cap, [&](int i) {
         bool in = false;
         if (i < N) {
             if (N == 4) in = true;
@@ -217,23 +214,11 @@ pnp_select_kernel(PnpArgs a)
                 in = pnp_is_inlier(s_h, a.fx, a.fy, a.cx, a.cy, o[0], o[1], o[2], m[0], m[1], a.thr_sq);
             }
         }
-        const unsigned bm = __ballot_sync(0xffffffffu, in);
-        if (lane == 0) s_warp[warp] = __popc(bm);
-        __syncthreads();
-        int off = s_base;
-        for (int w = 0; w < warp; ++w) off += s_warp[w];
-        if (in) inl[off + __popc(bm & ((1u << lane) - 1))] = i;
-        if (i < a.cap) mask[i] = in ? 1 : 0;
-        __syncthreads();
-        if (threadIdx.x == 0) {
-            int tot = 0;
-            for (int w = 0; w < 8; ++w) tot += s_warp[w];
-            s_base += tot;
-        }
-        __syncthreads();
-    }
+        mask[i] = in ? 1 : 0;
+        return in;
+    }, [&](int i, int o) { inl[o] = i; });
     if (threadIdx.x == 0) {
-        a.n_inliers[b] = s_base;
+        a.n_inliers[b] = M;
         a.ok[b] = 1;
         // RANSAC model (what cv2 falls back to / returns for N == 4)
         double* pose = a.pose + (size_t)b * 6;
@@ -786,6 +771,7 @@ pnp_fused_kernel(PnpArgs a, PoseBatchIO io)
 
     phase_stamp(a, b, 0);
     // ---- 1. status == 1 landmarks, in order (what `matched_pts[tracked]` does in the reference, :282-284) ----
+    // (written out rather than cta_compact: this kernel's register allocation is at its limit, <2> spills)
     if (tid == 0) F.base = 0;
     __syncthreads();
     if (io.lm_status) {
@@ -900,6 +886,7 @@ pnp_fused_kernel(PnpArgs a, PoseBatchIO io)
         for (int i = tid; i < a.cap; i += FUSED_T) mask[i] = 0;
         if (tid == 0) { a.n_inliers[b] = 0; a.ok[b] = 0; }
     } else {
+        // written out rather than cta_compact, as in step 1
         for (int base = 0; base < a.cap; base += FUSED_T) {
             const int i = base + tid;
             bool in = false;

@@ -527,59 +527,36 @@ struct SiftKpLess {
 
 #define SIFT_DEDUP_T 256
 // One CTA per frame of the chunk: the frame's run [lo, hi) of the sorted list, first of each (x, y, size, angle) group kept in
-// order (ballot + running base) at out[lo + rank]; the rest of the run is marked free.  Writes the kept keypoints in the
+// order (cta_compact) at out[lo + rank]; the rest of the run is marked free.  Writes the kept keypoints in the
 // caller's format (firstOctave = -1 undone: coordinates and size halved, octave - 1 in the low byte) at kp6[base + lo + rank],
 // and per frame the count and the first row.
 __global__ void __launch_bounds__(SIFT_DEDUP_T)
 sift_dedup_kernel(const SiftKp* __restrict__ sorted, int n, SiftKp* __restrict__ out, float* __restrict__ kp6, int base,
                   int* __restrict__ n_frame, int* __restrict__ first_row)
 {
-    __shared__ int s_warp[SIFT_DEDUP_T / 32];
-    __shared__ int s_lo, s_hi, s_base;
-    const int f = blockIdx.x, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    __shared__ int s_lo, s_hi;
+    const int f = blockIdx.x;
     if (threadIdx.x < 2) {   // lower bounds of f and f + 1
         const int key = f + threadIdx.x;
         int a = 0, b = n;
         while (a < b) { const int m = (a + b) >> 1; if (sorted[m].f < key) a = m + 1; else b = m; }
         if (threadIdx.x == 0) s_lo = a; else s_hi = a;
     }
-    if (threadIdx.x == 0) s_base = 0;
     __syncthreads();
     const int lo = s_lo, hi = s_hi;
-    for (int i0 = lo; i0 < hi; i0 += SIFT_DEDUP_T) {
-        const int i = i0 + threadIdx.x;
-        bool keep = false;
-        SiftKp k{};
-        if (i < hi) {
-            k = sorted[i];
-            keep = i == lo;
-            if (!keep) {
-                const SiftKp& p = sorted[i - 1];
-                keep = p.x != k.x || p.y != k.y || p.size != k.size || p.angle != k.angle;
-            }
-        }
-        const unsigned bm = __ballot_sync(0xffffffffu, keep);
-        if (lane == 0) s_warp[warp] = __popc(bm);
-        __syncthreads();
-        int o = s_base;
-        for (int w = 0; w < warp; ++w) o += s_warp[w];
-        o += __popc(bm & ((1u << lane) - 1));
-        if (keep) {
-            out[lo + o] = k;
-            const int oc = (k.octave_code & ~255) | ((k.octave_code - 1) & 255);
-            float* q = kp6 + (size_t)(base + lo + o) * 6;
-            q[0] = k.x * 0.5f; q[1] = k.y * 0.5f; q[2] = k.size * 0.5f; q[3] = k.angle; q[4] = k.response;
-            memcpy(&q[5], &oc, 4);
-        }
-        __syncthreads();
-        if (threadIdx.x == 0) {
-            int tot = 0;
-            for (int w = 0; w < SIFT_DEDUP_T / 32; ++w) tot += s_warp[w];
-            s_base += tot;
-        }
-        __syncthreads();
-    }
-    const int cnt = s_base;
+    const int cnt = cta_compact<SIFT_DEDUP_T>(hi - lo, [&](int j) {
+        if (j == 0) return true;
+        const SiftKp& p = sorted[lo + j - 1];
+        const SiftKp& k = sorted[lo + j];
+        return p.x != k.x || p.y != k.y || p.size != k.size || p.angle != k.angle;
+    }, [&](int j, int o) {
+        const SiftKp k = sorted[lo + j];
+        out[lo + o] = k;
+        const int oc = (k.octave_code & ~255) | ((k.octave_code - 1) & 255);
+        float* q = kp6 + (size_t)(base + lo + o) * 6;
+        q[0] = k.x * 0.5f; q[1] = k.y * 0.5f; q[2] = k.size * 0.5f; q[3] = k.angle; q[4] = k.response;
+        memcpy(&q[5], &oc, 4);
+    });
     for (int i = lo + cnt + threadIdx.x; i < hi; i += SIFT_DEDUP_T) out[i].f = -1;
     if (threadIdx.x == 0) { n_frame[f] = cnt; first_row[f] = base + lo; }
 }

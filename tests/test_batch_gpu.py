@@ -61,6 +61,39 @@ def test_batch_equals_per_call_path(wl, pinned):
             assert np.array_equal(o["pose"][s], np.concatenate([rv.ravel(), tv.ravel()]))
 
 
+def test_unfused_pose_path_equals_fused(wl):
+    """A landmark capacity above VO_PNP_FUSED_MAX_N (4096, csrc/pnp.cuh) runs the separate pose kernels (status compaction,
+    RANSAC, select, EPnP, mask scatter) instead of the fused one.  Against a twin at capacity 4096 stepped on the same data:
+    identical tracks, decisions and inliers; poses to rounding, since the two paths run different 12x12 Jacobi schedules."""
+    opts = workload.REFERENCE_OPTIONS["kitti"]
+    fused_max, n_steps = 4096, 3
+    order = workload.frame_order(wl.F, n_steps)
+    outs = {}
+    for L in (fused_max + 4, fused_max):
+        lm_pts = np.zeros((wl.F, wl.batch, L, 2), np.float32)
+        lm_obj = np.zeros((wl.F, wl.batch, L, 3), np.float32)
+        lm_pts[:, :, :wl.L], lm_obj[:, :, :wl.L] = wl.lm_pts, wl.lm_obj
+        sb = SequenceBatch(wl.batch, wl.h, wl.w, wl.K, win=opts["win"], max_level=opts["max_level"], criteria=opts["criteria"],
+                           pnp_iters=opts["pnp_iters"], pnp_reproj_err=opts["pnp_err"], pnp_conf=opts["pnp_conf"],
+                           max_landmarks=L, max_candidates=wl.Cn)
+        sb.prime(wl.frames[order[0]])
+        outs[L] = []
+        for t in range(n_steps):
+            f, g = order[t], order[t + 1]
+            o = sb.step(wl.frames[g], lm_pts[f], lm_obj[f], wl.n_lm[f], wl.cand_pts[f], wl.n_cand[f])
+            outs[L].append({k: v.copy() for k, v in o.items()})
+        sb.close()
+    for t in range(n_steps):
+        u, w = outs[fused_max + 4][t], outs[fused_max][t]
+        for s in range(wl.batch):
+            nl = int(wl.n_lm[order[t], s])
+            assert np.array_equal(u["lm_status"][s, :nl], w["lm_status"][s, :nl]), (t, s)
+            assert np.array_equal(u["inlier_mask"][s, :fused_max], w["inlier_mask"][s]) and not u["inlier_mask"][s, fused_max:].any(), (t, s)
+        assert u["pnp_ok"].all() and np.array_equal(u["pnp_ok"], w["pnp_ok"]) and np.array_equal(u["n_inliers"], w["n_inliers"]), t
+        d = np.abs(u["pose"] - w["pose"]).max()
+        assert d <= 1e-9, (t, d)
+
+
 def test_batch_vs_oracle_and_truth(wl):
     import oracle
     opts = workload.REFERENCE_OPTIONS["kitti"]
