@@ -254,6 +254,14 @@ typedef struct {
 
 int b200vo_batch_create(b200vo_ctx* ctx, int batch, const b200vo_batch_cfg* cfg, b200vo_batch** out);
 void b200vo_batch_destroy(b200vo_batch* b);
+/*
+ * Per-sequence camera intrinsics.  b200vo_batch_create gives every sequence cfg->K; this call gives each of the n_seq distinct
+ * sequences seqs[k] the camera matrix K[k] (double [n_seq][9], row-major), which the pose chain of every later step uses.
+ * K[k] must be a pinhole camera: fx, fy finite and > 0, cx, cy finite, skew and the other off-diagonal entries 0, last row
+ * (0, 0, 1).  Bad indices (out of range, repeated), n_seq < 1, null arrays or a bad K: B200VO_E_BADARG and nothing changes.
+ * Synchronous (waits for the step in flight); touches nothing but the listed sequences' intrinsics.
+ */
+int b200vo_batch_set_intrinsics(b200vo_batch* b, int n_seq, const int32_t* seqs, const double* K);
 /* Upload the first frame of every sequence (frames: batch x rows x cols, tight). */
 int b200vo_batch_prime(b200vo_batch* b, const uint8_t* frames);
 /*
@@ -337,6 +345,12 @@ typedef struct {
 
 int b200vo_loop_create(b200vo_ctx* ctx, int batch, const b200vo_loop_cfg* cfg, b200vo_loop** out);
 void b200vo_loop_destroy(b200vo_loop* lp);
+/* Per-sequence camera intrinsics of the loop, as b200vo_batch_set_intrinsics: b200vo_loop_create gives every sequence
+ * cfg->batch.K; afterwards sequence seqs[k] is tracked, posed, triangulated and bootstrapped with K[k] (double [n_seq][9]).
+ * The state, status and frames of a sequence are not touched: a caller who hands a slot to another camera sets its K just
+ * before b200vo_loop_load or b200vo_loop_bootstrap of that slot.  Same validation (B200VO_E_BADARG, nothing changes).
+ * Synchronous. */
+int b200vo_loop_set_intrinsics(b200vo_loop* lp, int n_seq, const int32_t* seqs, const double* K);
 /* State of sequence `seq` after its bootstrap (host arrays): frame uint8 (rows,cols) tight = the current frame;
  * lm float32 (n_lm,3) + lm_kp float32 (n_lm,2); keys / first_keys float32 (n_cand,2) + first_pose int32 (n_cand)
  * = potential_keys / potential_first_keys / potential_transforms; poses double (n_poses,12) = self.transforms as

@@ -21,6 +21,36 @@ def _p(a, t):
     return a.ctypes.data_as(t)
 
 
+def _batch_K(K, batch):
+    """K of a batch constructor: (3, 3) for every sequence, or (batch, 3, 3), one per sequence.  -> (the (3, 3) matrix that goes
+    into the config, the (batch, 3, 3) rows to set afterwards or None)."""
+    K = np.asarray(K, np.float64)
+    if K.shape == (3, 3):
+        return K, None
+    if K.shape == (batch, 3, 3):
+        return K[0], np.ascontiguousarray(K)
+    raise ValueError(f"K must be (3, 3) or (batch = {batch}, 3, 3), got {K.shape}")
+
+
+def _pinhole(K) -> bool:
+    """What b200vo_*_set_intrinsics accepts (checked here where a refusal must come before another call)."""
+    return bool(np.isfinite(K).all() and K[0, 0] > 0 and K[1, 1] > 0 and K[0, 1] == 0 and K[1, 0] == 0 and K[2, 0] == 0
+                and K[2, 1] == 0 and K[2, 2] == 1)
+
+
+def _set_intrinsics(ctx, fn, h, batch, seqs, K, what):
+    """Shared body of SequenceBatch / VOBatch.set_intrinsics."""
+    seqs = np.ascontiguousarray(seqs, np.int32).reshape(-1)
+    K = np.ascontiguousarray(K, np.float64)
+    if K.shape != (len(seqs), 3, 3):
+        raise ValueError(f"K must be (len(seqs) = {len(seqs)}, 3, 3), got {K.shape}")
+    rc = fn(h, len(seqs), _p(seqs, c_i32p), _p(K, c_f64p))
+    if rc == -1:
+        raise ValueError(f"{what}: {ctx.last_error()}")
+    if rc != 0:
+        raise _lib.B200VOError(f"{what} failed ({rc}): {ctx.last_error()}")
+
+
 class _PinnedBlock:
     """Owner of one b200vo_host_alloc block.  The numpy arrays carved from it keep it alive (it hangs off the
     ctypes buffer that is the arrays' base), so a result array that outlives its SequenceBatch -- e.g.
@@ -62,7 +92,8 @@ class SequenceBatch:
         cfg.crit_type, cfg.crit_max_count, cfg.crit_eps = int(criteria[0]), int(criteria[1]), float(criteria[2])
         cfg.min_eig_thr = float(min_eig_thr)
         cfg.pnp_iters, cfg.pnp_reproj_err, cfg.pnp_conf = int(pnp_iters), float(pnp_reproj_err), float(pnp_conf)
-        Kf = np.asarray(K, np.float64).reshape(9)
+        K, K_rows = _batch_K(K, self.batch)
+        Kf = K.reshape(9)
         for i in range(9):
             cfg.K[i] = float(Kf[i])
         cfg.max_landmarks, cfg.max_candidates = self.L, self.Cn
@@ -72,6 +103,8 @@ class SequenceBatch:
         if rc != 0:
             raise _lib.B200VOError(f"b200vo_batch_create failed ({rc}): {self.ctx.last_error()}")
         self.h = h
+        if K_rows is not None:
+            self.set_intrinsics(np.arange(self.batch), K_rows)
         # host outputs (reused, page-locked so that step() reads them back without a staging copy)
         b, L, Cn = self.batch, self.L, self.Cn
         self.lm_next = self.pinned_empty((b, L, 2), np.float32)
@@ -105,6 +138,12 @@ class SequenceBatch:
     def _chk(self, rc, what):
         if rc != 0:
             raise _lib.B200VOError(f"{what} failed ({rc}): {self.ctx.last_error()}")
+
+    def set_intrinsics(self, seqs, K):
+        """Give the distinct sequences ``seqs`` the camera matrices ``K`` (len(seqs), 3, 3); every later step poses them with
+        their own K.  A K must be a pinhole camera: fx, fy finite and > 0, cx, cy finite, zero skew and other off-diagonal
+        entries, last row (0, 0, 1).  Bad shapes, indices or matrices raise ValueError and change nothing.  Synchronous."""
+        _set_intrinsics(self.ctx, self.ctx.lib.b200vo_batch_set_intrinsics, self.h, self.batch, seqs, K, "b200vo_batch_set_intrinsics")
 
     def pinned_empty(self, shape, dtype) -> np.ndarray:
         """numpy array in page-locked host memory (b200vo_host_alloc): DMA'd in place by step()."""
@@ -189,7 +228,7 @@ def _loop_cfg(rows, cols, K, options, max_landmarks, max_candidates, max_frames)
     bc.crit_type, bc.crit_max_count, bc.crit_eps = int(o['criteria'][0]), int(o['criteria'][1]), float(o['criteria'][2])
     bc.min_eig_thr = 1e-4                          # cv2.calcOpticalFlowPyrLK's default (the reference passes none)
     bc.pnp_iters, bc.pnp_reproj_err, bc.pnp_conf = int(o['PnP_iterations']), float(o['PnP_error']), float(o['PnP_conf'])
-    Kf = np.asarray(K, np.float64).reshape(9)
+    Kf = np.asarray(K, np.float64).reshape(9)   # the (3, 3) K of every sequence (per-sequence rows: VOBatch.set_intrinsics)
     for i in range(9):
         bc.K[i] = float(Kf[i])
     bc.max_landmarks, bc.max_candidates = int(max_landmarks), int(max_candidates)
@@ -213,7 +252,10 @@ class VOBatch:
     and ``first_pose`` int32 (n_cand,), and ``poses`` float64 (n_poses,12) = ``self.transforms`` as (R_CW | t_CW).
     A sequence that cannot follow the reference's data flow stops with one of the status codes below and stays as it
     is until it is loaded again.  ``bootstrap`` runs the reference's bootstrap for any subset of the sequences on the
-    device instead of ``load``; a sequence whose bootstrap finds no essential matrix gets ``NO_BOOTSTRAP``."""
+    device instead of ``load``; a sequence whose bootstrap finds no essential matrix gets ``NO_BOOTSTRAP``.
+
+    ``K`` is the camera matrix of every sequence, (3, 3), or one per sequence, (batch, 3, 3).  ``set_intrinsics`` (or the
+    ``K`` argument of ``load`` / ``bootstrap``) gives a slot another camera, e.g. when it is handed to a new sequence."""
 
     OK, IDLE, FEW_POINTS, PNP_FAILED, OVERFLOW, DETECT_LIMIT, NO_BOOTSTRAP = range(7)
 
@@ -223,12 +265,15 @@ class VOBatch:
         self.batch, self.rows, self.cols = int(batch), int(rows), int(cols)
         self.L, self.Cn, self.P = int(max_landmarks), int(max_candidates), int(max_frames)
         self.options = options
+        K, K_rows = _batch_K(K, self.batch)
         self.cfg = _loop_cfg(rows, cols, K, options, max_landmarks, max_candidates, max_frames)
         h = C.c_void_p()
         rc = self.ctx.lib.b200vo_loop_create(self.ctx.h, self.batch, C.byref(self.cfg), C.byref(h))
         if rc != 0:
             raise _lib.B200VOError(f"b200vo_loop_create failed ({rc}): {self.ctx.last_error()}")
         self.h = h
+        if K_rows is not None:
+            self.set_intrinsics(np.arange(self.batch), K_rows)
         b = self.batch
         self._res = dict(status=self.pinned_empty((b,), np.int32), n_inliers=self.pinned_empty((b,), np.int32),
                          n_lm=self.pinned_empty((b,), np.int32), n_cand=self.pinned_empty((b,), np.int32),
@@ -263,9 +308,18 @@ class VOBatch:
         """(n_sets, batch, rows, cols) uint8 array in page-locked memory, for submit_frames() and step()."""
         return self.pinned_empty((n_sets, self.batch, self.rows, self.cols), np.uint8)
 
-    def load(self, seq: int, frame: np.ndarray, state: dict):
+    def set_intrinsics(self, seqs, K):
+        """Give the distinct sequences ``seqs`` the camera matrices ``K`` (len(seqs), 3, 3): every later step and bootstrap of
+        those sequences tracks, poses and triangulates with their own K.  A K must be a pinhole camera: fx, fy finite and > 0,
+        cx, cy finite, zero skew and other off-diagonal entries, last row (0, 0, 1).  The sequences' states, status and frames
+        are not touched: to hand a slot to a sequence of another camera, set its K just before ``load`` or ``bootstrap`` (or
+        pass ``K`` to them).  Bad shapes, indices or matrices raise ValueError and change nothing.  Synchronous."""
+        _set_intrinsics(self.ctx, self.ctx.lib.b200vo_loop_set_intrinsics, self.h, self.batch, seqs, K, "b200vo_loop_set_intrinsics")
+
+    def load(self, seq: int, frame: np.ndarray, state: dict, K=None):
         """Set sequence ``seq`` to ``state`` (see the class docstring) with ``frame`` as its current frame; its status
-        becomes OK.  Out-of-range counts or first_pose values raise ValueError and change nothing."""
+        becomes OK.  ``K`` (3, 3): the sequence's camera from now on (``set_intrinsics`` first).  Out-of-range counts or
+        first_pose values raise ValueError and change nothing."""
         f = np.ascontiguousarray(frame, np.uint8)
         if f.shape != (self.rows, self.cols):
             raise ValueError(f"frame must be ({self.rows}, {self.cols}) uint8")
@@ -277,24 +331,33 @@ class VOBatch:
         poses = np.ascontiguousarray(state['poses'], np.float64).reshape(-1, 12)
         if len(kp) != len(lm) or len(fk) != len(keys) or len(fp) != len(keys):
             raise ValueError("lm / lm_kp and keys / first_keys / first_pose must have one row per point")
+        if K is not None:
+            K = np.asarray(K, np.float64)
+            if K.shape != (3, 3) or not _pinhole(K):
+                raise ValueError("K must be a (3, 3) pinhole camera matrix (see set_intrinsics)")
         self._chk(self.ctx.lib.b200vo_loop_load(self.h, int(seq), _p(f, c_u8p), _p(lm, c_f32p), _p(kp, c_f32p), len(lm),
                                                 _p(keys, c_f32p), _p(fk, c_f32p), _p(fp, c_i32p), len(keys), _p(poses, c_f64p),
                                                 len(poses)), "b200vo_loop_load")
+        if K is not None:   # after the load, which is the call that can still refuse
+            self.set_intrinsics([seq], K[None])
 
-    def bootstrap(self, frames0, frames1, seqs=None) -> dict:
+    def bootstrap(self, frames0, frames1, seqs=None, K=None) -> dict:
         """The reference's bootstrap (``initialization``) on the device for the sequences ``seqs`` (distinct indices; None:
         every sequence) from their two bootstrap frames ``frames0`` / ``frames1`` (len(seqs), rows, cols) uint8, with the
         ratio ``options['feature_ratio']``.  A sequence that succeeds ends up exactly as ``load(s, frames1[k],
         initial_state(K, options, *match_bootstrap_frames(frames0[k], frames1[k], ratio)))`` leaves it.  Returns int32
         arrays (len(seqs),): ``status`` (OK, NO_BOOTSTRAP or OVERFLOW), ``num_pts`` (the essential-matrix inlier count),
         ``n_lm`` and ``n_cand``.  A failing sequence keeps its state and is skipped by ``step`` until it is loaded or
-        bootstrapped again.  Bad indices or frame shapes raise ValueError and change nothing.  Synchronous."""
+        bootstrapped again.  ``K`` (len(seqs), 3, 3): the listed sequences' cameras from now on (``set_intrinsics`` first).
+        Bad indices, frame shapes or K raise ValueError and change nothing.  Synchronous."""
         seqs = np.arange(self.batch, dtype=np.int32) if seqs is None else np.ascontiguousarray(seqs, np.int32).reshape(-1)
         f0 = np.ascontiguousarray(frames0, np.uint8)
         f1 = np.ascontiguousarray(frames1, np.uint8)
         shape = (len(seqs), self.rows, self.cols)
         if f0.shape != shape or f1.shape != shape:
             raise ValueError(f"frames0 and frames1 must be {shape} uint8")
+        if K is not None:
+            self.set_intrinsics(seqs, K)
         n = len(seqs)
         out = {k: np.zeros(max(n, 1), np.int32) for k in ('status', 'num_pts', 'n_lm', 'n_cand')}
         self._chk(self.ctx.lib.b200vo_loop_bootstrap(self.h, n, _p(seqs, c_i32p), _p(f0, c_u8p), _p(f1, c_u8p),

@@ -111,8 +111,38 @@ extern "C" int b200vo_batch_create(b200vo_ctx* ctx, int batch, const b200vo_batc
     B->inliers = (int*)p; p += b_i;
     B->c_mask = p; p += b_m;
     B->pnp_ws = p;
+    // every sequence starts with cfg->K
+    B->intr_host.resize(batch);
+    vo_intrinsics_row(B->intr_host[0], cfg->K, VO_BOOT_EMAT_THR);
+    for (int k = 1; k < batch; ++k) B->intr_host[k] = B->intr_host[0];
+    rc = vo_reserve(ctx, B->intr_buf, (size_t)batch * sizeof(VoIntrinsics));
+    if (!rc) {
+        cudaError_t e = cudaMemcpyAsync(B->intr_buf.p, B->intr_host.data(), (size_t)batch * sizeof(VoIntrinsics), cudaMemcpyHostToDevice, ctx->stream);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+        if (e != cudaSuccess) rc = vo_cuda_fail(ctx, e, "b200vo_batch_create: intrinsics upload");
+    }
+    if (rc) { b200vo_batch_destroy(B); return rc; }
+    B->intr = (const VoIntrinsics*)B->intr_buf.p;
     *out = B;
     return 0;
+}
+
+int batch_set_intrinsics(b200vo_batch* B, int n_seq, const int32_t* seqs, const double* K)
+{
+    b200vo_ctx* ctx = B->ctx;
+    std::vector<VoIntrinsics> rows = B->intr_host;
+    VO_TRY(vo_intrinsics_set(ctx, B->batch, n_seq, seqs, K, VO_BOOT_EMAT_THR, rows.data()));
+    VO_CUDA(ctx, cudaSetDevice(ctx->device));
+    VO_CUDA(ctx, cudaStreamSynchronize(ctx->stream));   // no step in flight reads the rows (every stream of a step joins the ctx stream)
+    VO_CUDA(ctx, cudaMemcpyAsync(B->intr_buf.p, rows.data(), rows.size() * sizeof(VoIntrinsics), cudaMemcpyHostToDevice, ctx->stream));
+    VO_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    B->intr_host.swap(rows);
+    return 0;
+}
+
+extern "C" int b200vo_batch_set_intrinsics(b200vo_batch* B, int n_seq, const int32_t* seqs, const double* K)
+{
+    return B ? batch_set_intrinsics(B, n_seq, seqs, K) : B200VO_E_BADARG;
 }
 
 __global__ void trace_stamp_kernel(unsigned long long* dst)
@@ -177,7 +207,7 @@ extern "C" void b200vo_batch_destroy(b200vo_batch* B)
     kill_stream(B->io_stream);
     kill_stream(B->pose_stream);
     for (auto& s : B->slabs) if (s.p) cudaFree(s.p);
-    for (DevBuf* d : {&B->raw, &B->raw_pre, &B->pts_in, &B->outs, &B->work, &B->gftt_ws}) if (d->p) cudaFree(d->p);
+    for (DevBuf* d : {&B->raw, &B->raw_pre, &B->pts_in, &B->outs, &B->work, &B->gftt_ws, &B->intr_buf}) if (d->p) cudaFree(d->p);
     for (auto& e : B->q_ev) kill_event(e);
     for (auto& e : B->chunk_ev) kill_event(e);
     for (auto& e : B->copy_ev) kill_event(e);
@@ -341,9 +371,12 @@ static int batch_pose(b200vo_batch* B, cudaStream_t stream, const float* lm_obj,
     PnpArgs a{};
     a.batch = B->batch; a.cap = c.max_landmarks; a.iters = c.pnp_iters;
     a.obj = B->c_obj; a.img = B->c_img; a.n = B->c_n;
-    a.fx = c.K[0]; a.fy = c.K[4]; a.cx = c.K[2]; a.cy = c.K[5];
+    a.intr = B->intr;
     a.thr_sq = (float)((double)c.pnp_reproj_err * (double)c.pnp_reproj_err);
     a.conf = c.pnp_conf;
+    // the ctx's table of cv2 random numbers moves when a longer draw grows it (the bootstrap's E-RANSAC does): look it up
+    // at every step rather than keeping the address of creation time (no synchronisation unless it has to grow)
+    VO_TRY(vo_rng_table(ctx, B->n_raw, &B->rng));
     a.rng_raw = B->rng; a.n_raw = B->n_raw;
     a.inliers = B->inliers; a.mask = B->c_mask; a.pose = pose;
     vo_pnp_carve_workspace(a, B->pnp_ws);

@@ -43,6 +43,10 @@ struct b200vo_batch {
     void* pnp_ws;
     const uint32_t* rng; int n_raw;
     bool primed;
+    // the camera of every sequence (b200vo_batch_set_intrinsics): device rows read by the kernels, host mirror of them
+    DevBuf intr_buf;
+    const VoIntrinsics* intr = nullptr;
+    std::vector<VoIntrinsics> intr_host;
     // host-input path: frames arrive chunk by chunk on a copy stream while earlier chunks are tracked
     cudaStream_t chunk_stream[B200VO_BATCH_STREAMS] = {};  // chunk k: H2D -> pyramid -> KLT on stream k % STREAMS
     cudaEvent_t chunk_ev[B200VO_BATCH_CHUNKS] = {};
@@ -74,3 +78,5 @@ int batch_track_pose_overlapped(b200vo_batch* B, const uint8_t* frames_dev, cons
                                 uint8_t* pnp_ok, uint8_t* inlier_mask, int* n_inliers, cudaEvent_t obj_ready,
                                 cudaEvent_t cand_ready = nullptr);
 int batch_finish(b200vo_batch* B);
+// Validates the (index, K) pairs and, only when all are valid, waits for the work in flight and uploads the new rows (synchronous)
+int batch_set_intrinsics(b200vo_batch* B, int n_seq, const int32_t* seqs, const double* K);

@@ -17,7 +17,7 @@ static int pnp_run(b200vo_ctx* ctx, const float* obj, const float* img, int n, c
     VO_CUDA(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
     PnpArgs a{};
     a.batch = 1; a.cap = n; a.iters = iters;
-    a.fx = K[0]; a.fy = K[4]; a.cx = K[2]; a.cy = K[5];
+    VO_TRY(vo_intrinsics_uniform(ctx, K, VO_BOOT_EMAT_THR, 1, &a.intr));   // the batch of one
     a.thr_sq = (float)((double)reproj_err * (double)reproj_err);
     a.conf = conf;
     a.full_counts = counts_out != nullptr;
@@ -119,7 +119,7 @@ extern "C" int b200vo_solve_pnp_ransac_p3p_dev(b200vo_ctx* ctx, const float* obj
     VO_CUDA(ctx, cudaSetDevice(ctx->device));
     PnpArgs a{};
     a.batch = 1; a.cap = n; a.iters = iters;
-    a.fx = K[0]; a.fy = K[4]; a.cx = K[2]; a.cy = K[5];
+    VO_TRY(vo_intrinsics_uniform(ctx, K, VO_BOOT_EMAT_THR, 1, &a.intr));   // the batch of one
     a.thr_sq = (float)((double)reproj_err * (double)reproj_err);
     a.conf = conf;
     a.n_raw = 8 * iters + 256;
@@ -148,7 +148,7 @@ extern "C" int b200vo_debug_pose_phases(b200vo_ctx* ctx, const float* obj_dev, c
     VO_CUDA(ctx, cudaSetDevice(ctx->device));
     PnpArgs a{};
     a.batch = 1; a.cap = n; a.iters = iters < 1 ? 1 : iters;
-    a.fx = K[0]; a.fy = K[4]; a.cx = K[2]; a.cy = K[5];
+    VO_TRY(vo_intrinsics_uniform(ctx, K, VO_BOOT_EMAT_THR, 1, &a.intr));   // the batch of one
     a.thr_sq = (float)((double)reproj_err * (double)reproj_err);
     a.conf = conf;
     a.n_raw = 8 * a.iters + 256;

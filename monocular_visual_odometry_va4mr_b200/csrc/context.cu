@@ -1,6 +1,7 @@
 // Context, buffer pool and error plumbing of libb200vo.so.
 #include "internal.cuh"
 #include "tma.cuh"
+#include <cmath>
 #include <cstdarg>
 
 int vo_set_err(b200vo_ctx* ctx, int code, const char* fmt, ...)
@@ -50,6 +51,55 @@ int vo_reserve_pinned(b200vo_ctx* ctx, size_t bytes)
     return 0;
 }
 
+bool vo_intrinsics_valid(const double K[9])
+{
+    if (!K) return false;
+    const bool focal = std::isfinite(K[0]) && K[0] > 0 && std::isfinite(K[4]) && K[4] > 0;
+    const bool centre = std::isfinite(K[2]) && std::isfinite(K[5]);
+    const bool zeros = K[1] == 0 && K[3] == 0 && K[6] == 0 && K[7] == 0 && K[8] == 1;
+    return focal && centre && zeros;
+}
+
+void vo_intrinsics_row(VoIntrinsics& r, const double K[9], double emat_thr)
+{
+    r = VoIntrinsics{};
+    r.fx = K[0]; r.fy = K[4]; r.cx = K[2]; r.cy = K[5];
+    for (int k = 0; k < 9; ++k) r.K[k] = K[k];
+    const double Ki[9] = {1.0 / K[0], 0, -K[2] / K[0], 0, 1.0 / K[4], -K[5] / K[4], 0, 0, 1};
+    for (int k = 0; k < 9; ++k) r.Ki[k] = Ki[k];
+    const double t = emat_thr / ((r.fx + r.fy) / 2);
+    r.emat_thr_sq = (float)(t * t);
+}
+
+int vo_intrinsics_uniform(b200vo_ctx* ctx, const double K[9], double emat_thr, int n, const VoIntrinsics** d_rows)
+{
+    std::vector<VoIntrinsics> h(n > 0 ? n : 1);
+    vo_intrinsics_row(h[0], K, emat_thr);
+    for (size_t s = 1; s < h.size(); ++s) h[s] = h[0];
+    VO_TRY(vo_reserve(ctx, ctx->d_intr, h.size() * sizeof(VoIntrinsics)));
+    VO_CUDA(ctx, cudaMemcpyAsync(ctx->d_intr.p, h.data(), h.size() * sizeof(VoIntrinsics), cudaMemcpyHostToDevice, ctx->stream));
+    *d_rows = (const VoIntrinsics*)ctx->d_intr.p;
+    return 0;
+}
+
+int vo_intrinsics_set(b200vo_ctx* ctx, int batch, int n_seq, const int32_t* seqs, const double* K, double emat_thr,
+                      VoIntrinsics* rows)
+{
+    if (n_seq < 1 || n_seq > batch) return vo_set_err(ctx, B200VO_E_BADARG, "n_seq = %d is outside [1, batch = %d]", n_seq, batch);
+    if (!seqs || !K) return vo_set_err(ctx, B200VO_E_BADARG, "null array");
+    std::vector<char> seen(batch, 0);
+    for (int k = 0; k < n_seq; ++k) {
+        if (seqs[k] < 0 || seqs[k] >= batch)
+            return vo_set_err(ctx, B200VO_E_BADARG, "seqs[%d] = %d is outside [0, batch = %d)", k, seqs[k], batch);
+        if (seen[seqs[k]]++) return vo_set_err(ctx, B200VO_E_BADARG, "sequence %d is listed twice", seqs[k]);
+        if (!vo_intrinsics_valid(K + 9 * k))
+            return vo_set_err(ctx, B200VO_E_BADARG, "K[%d] is not a camera matrix: fx, fy finite and > 0, cx, cy finite, "
+                                                    "skew 0, last row (0, 0, 1)", k);
+    }
+    for (int k = 0; k < n_seq; ++k) vo_intrinsics_row(rows[seqs[k]], K + 9 * k, emat_thr);
+    return 0;
+}
+
 extern "C" int b200vo_version(int* sm_arch)
 {
     if (sm_arch) *sm_arch = 100;
@@ -90,6 +140,7 @@ extern "C" void b200vo_destroy(b200vo_ctx* ctx)
     for (auto& b : ctx->d_scratch) if (b.p) cudaFree(b.p);
     for (auto& s : ctx->slots) if (s.slab.p) cudaFree(s.slab.p);
     if (ctx->d_rng.p) cudaFree(ctx->d_rng.p);
+    if (ctx->d_intr.p) cudaFree(ctx->d_intr.p);
     if (ctx->d_sift.p) cudaFree(ctx->d_sift.p);
     for (DevBuf* b : {&ctx->d_sift_out[0], &ctx->d_sift_out[1], &ctx->d_sift_sort}) if (b->p) cudaFree(b->p);
     if (ctx->d_klt_queue.p) cudaFree(ctx->d_klt_queue.p);

@@ -389,8 +389,7 @@ struct EmatArgs {
     int n, iters;                          // n < 0: each sequence's count is n_dev[s] (emat_seq reads it)
     int cap;                               // point slots per sequence
     const float* p1; const float* p2;     // [n][2] pixels
-    double fx, fy, cx, cy;
-    float thr_sq;
+    const VoIntrinsics* intr;              // [nseq] camera and Sampson threshold of each set
     double conf;
     double* x1; double* x2;               // [n][2] normalised
     int* n_dev;                            // [1] = n
@@ -414,7 +413,7 @@ __device__ __forceinline__ EmatArgs emat_seq(const EmatArgs& A, int s)
     const size_t pc = (size_t)s * A.cap, ic = (size_t)s * A.iters;
     a.p1 += 2 * pc; a.p2 += 2 * pc; a.x1 += 2 * pc; a.x2 += 2 * pc; a.mask += pc;
     a.samples += 5 * ic; a.models += ic * EM_MAXM * 9; a.nmodels += ic; a.counts += ic * EM_MAXM;
-    a.E += 9 * s; a.result += 4 * s; a.state += 4 * s; a.n_dev += s; a.flags += s;
+    a.E += 9 * s; a.result += 4 * s; a.state += 4 * s; a.n_dev += s; a.flags += s; a.intr += s;
     if (A.n < 0) a.n = *a.n_dev;
     return a;
 }
@@ -429,8 +428,9 @@ emat_normalize_kernel(EmatArgs A)
         *a.flags = 0;
     }
     if (i >= a.n) return;
-    a.x1[2 * i] = ((double)a.p1[2 * i] - a.cx) / a.fx; a.x1[2 * i + 1] = ((double)a.p1[2 * i + 1] - a.cy) / a.fy;
-    a.x2[2 * i] = ((double)a.p2[2 * i] - a.cx) / a.fx; a.x2[2 * i + 1] = ((double)a.p2[2 * i + 1] - a.cy) / a.fy;
+    const VoIntrinsics& c = *a.intr;
+    a.x1[2 * i] = ((double)a.p1[2 * i] - c.cx) / c.fx; a.x1[2 * i + 1] = ((double)a.p1[2 * i + 1] - c.cy) / c.fy;
+    a.x2[2 * i] = ((double)a.p2[2 * i] - c.cx) / c.fx; a.x2[2 * i + 1] = ((double)a.p2[2 * i + 1] - c.cy) / c.fy;
 }
 
 __global__ void __launch_bounds__(EMW_WARPS * 32)
@@ -484,9 +484,10 @@ emat_score_kernel(EmatArgs A)
     double ax = 0, ay = 0, bx = 0, by = 0;
     if (live) { ax = a.x1[2 * i]; ay = a.x1[2 * i + 1]; bx = a.x2[2 * i]; by = a.x2[2 * i + 1]; }
     const int lane = threadIdx.x & 31;
+    const float thr_sq = a.intr->emat_thr_sq;
     for (int s = 0; s < ns; ++s)
         for (int m = 0; m < s_nm[s]; ++m) {
-            const bool in = live && sampson_inlier(s_E + (s * EM_MAXM + m) * 9, ax, ay, bx, by, a.thr_sq);
+            const bool in = live && sampson_inlier(s_E + (s * EM_MAXM + m) * 9, ax, ay, bx, by, thr_sq);
             const unsigned bm = __ballot_sync(0xffffffffu, in);
             if (lane == 0 && bm) atomicAdd(a.counts + (it0 + s) * EM_MAXM + m, __popc(bm));
         }
@@ -532,8 +533,9 @@ emat_finish_kernel(EmatArgs A)
     }
     if (threadIdx.x < 9) { s_E[threadIdx.x] = a.models[(size_t)win * 9 + threadIdx.x]; a.E[threadIdx.x] = s_E[threadIdx.x]; }
     __syncthreads();
+    const float thr_sq = a.intr->emat_thr_sq;
     for (int i = threadIdx.x; i < a.n; i += blockDim.x)
-        a.mask[i] = (a.n == 5) ? 1 : (sampson_inlier(s_E, a.x1[2 * i], a.x1[2 * i + 1], a.x2[2 * i], a.x2[2 * i + 1], a.thr_sq) ? 1 : 0);
+        a.mask[i] = (a.n == 5) ? 1 : (sampson_inlier(s_E, a.x1[2 * i], a.x1[2 * i + 1], a.x2[2 * i], a.x2[2 * i + 1], thr_sq) ? 1 : 0);
 }
 
 int vo_rng_table(b200vo_ctx* ctx, int n, const uint32_t** d_table);
@@ -586,15 +588,14 @@ static int emat_launch(b200vo_ctx* ctx, EmatArgs& a, int nseq, int max_n, bool d
     return 0;
 }
 
-int vo_emat_batch(b200vo_ctx* ctx, const float* p1, const float* p2, int cap, const int* n_dev, int max_n, int nseq, const double K[9],
-                  double prob, double thr, int max_iters, double* E_dev, uint8_t* mask_dev, int* result_dev, int* flags_dev)
+int vo_emat_batch(b200vo_ctx* ctx, const float* p1, const float* p2, int cap, const int* n_dev, int max_n, int nseq,
+                  const VoIntrinsics* intr_dev, double prob, int max_iters, double* E_dev, uint8_t* mask_dev, int* result_dev,
+                  int* flags_dev)
 {
     const int iters = max_iters > 1 ? max_iters : 1;
     EmatArgs a{};
     a.n = -1; a.iters = iters; a.cap = cap;
-    a.fx = K[0]; a.fy = K[4]; a.cx = K[2]; a.cy = K[5];
-    const double t = thr / ((a.fx + a.fy) / 2);
-    a.thr_sq = (float)(t * t);
+    a.intr = intr_dev;
     a.conf = prob;
     const size_t ns = nseq;
     const size_t b_x = vo_align(ns * cap * 16, 256), b_s = vo_align(ns * iters * 5 * 4, 256), b_m = vo_align(ns * iters * EM_MAXM * 9 * 8, 256);
@@ -629,9 +630,7 @@ static int emat_run(b200vo_ctx* ctx, const float* p1, const float* p2, int n, co
     const int iters = max_iters > 1 ? max_iters : 1;
     EmatArgs a{};
     a.n = n; a.iters = iters; a.cap = n;
-    a.fx = K[0]; a.fy = K[4]; a.cx = K[2]; a.cy = K[5];
-    const double t = thr / ((a.fx + a.fy) / 2);
-    a.thr_sq = (float)(t * t);
+    VO_TRY(vo_intrinsics_uniform(ctx, K, thr, 1, &a.intr));   // the batch of one
     a.conf = prob;
     a.full = samples != nullptr;
     const size_t b_p = vo_align((size_t)n * 8, 256), b_x = vo_align((size_t)n * 16, 256);

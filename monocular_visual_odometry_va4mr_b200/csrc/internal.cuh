@@ -49,6 +49,28 @@ struct FrameSlot {
     bool valid = false;
 };
 
+// One sequence's camera as every kernel reads it: a device array of [batch] rows per batch object
+// (b200vo_batch_set_intrinsics / b200vo_loop_set_intrinsics), a one-row array for the one-call entry points.  Filled on
+// the host by vo_intrinsics_row in exactly the expressions the kernels used when K was a scalar argument, so a sequence
+// with a given K sees the same bits whatever the rest of its batch uses.
+struct VoIntrinsics {
+    double fx, fy, cx, cy;     // K[0], K[4], K[2], K[5]
+    double K[9], Ki[9];        // the triangulation's K and its inverse
+    float emat_thr_sq;         // E-RANSAC: (float)((thr / ((fx + fy) / 2))^2), Sampson error bound in normalised coordinates
+};
+#define VO_BOOT_EMAT_THR 1.0   // the bootstrap's findEssentialMat threshold (pixels, :308)
+
+// K is a pinhole camera matrix: fx, fy finite and > 0, cx, cy finite, skew and the other off-diagonal entries 0, last row (0, 0, 1)
+bool vo_intrinsics_valid(const double K[9]);
+void vo_intrinsics_row(VoIntrinsics& r, const double K[9], double emat_thr);
+// The single-K entry points: n identical rows of K in the ctx's own buffer, uploaded on the ctx stream (pageable source,
+// staged before the call returns, so the upload never waits for the device)
+int vo_intrinsics_uniform(b200vo_ctx* ctx, const double K[9], double emat_thr, int n, const VoIntrinsics** d_rows);
+// Validates the n_seq (index, K) pairs of a set_intrinsics call against [0, batch) and fills rows[seqs[k]] of the host mirror
+// `rows` ([batch]); nothing is written unless every pair is valid
+int vo_intrinsics_set(b200vo_ctx* ctx, int batch, int n_seq, const int32_t* seqs, const double* K, double emat_thr,
+                      VoIntrinsics* rows);
+
 struct b200vo_ctx {
     int device = 0;
     cudaStream_t stream = nullptr;
@@ -71,6 +93,7 @@ struct b200vo_ctx {
     DevBuf d_sift_sort;      // SIFT keypoint sort scratch
     DevBuf d_rng;            // raw cv::RNG stream (uint32)
     int n_rng = 0;
+    DevBuf d_intr;           // the one-row intrinsics array of the one-call entry points (vo_intrinsics_one)
     // tensor-map encode entry point (driver API, fetched lazily)
     void* encode_tiled = nullptr;
 };

@@ -90,6 +90,7 @@ __device__ __forceinline__ void triangulate_one(const TriArgs& a, int i)
 __device__ __forceinline__ TriArgs tri_sequence(const TriBatchArgs& b, int s)
 {
     TriArgs a = b.common;
+    a.K = b.intr[s].K; a.Ki = b.intr[s].Ki;
     const size_t o = (size_t)s * b.cap;
     a.n = min(max(b.n[s], 0), b.cap);
     a.n_poses = min(max(b.n_poses[s], 0), b.pose_cap);
@@ -147,11 +148,8 @@ min_distance_batch_kernel(const float2* __restrict__ pts, const int* __restrict_
     if (lane == 0) valid[(size_t)s * n_cap + i] = ok ? 1 : 0;
 }
 
-void vo_tri_common(TriArgs& c, const double K[9], double min_dist, double max_dist, double min_angle_deg, int min_frames)
+void vo_tri_common(TriArgs& c, double min_dist, double max_dist, double min_angle_deg, int min_frames)
 {
-    for (int k = 0; k < 9; ++k) c.K[k] = K[k];
-    const double Ki[9] = {1.0 / K[0], 0, -K[2] / K[0], 0, 1.0 / K[4], -K[5] / K[4], 0, 0, 1};
-    for (int k = 0; k < 9; ++k) c.Ki[k] = Ki[k];
     c.min_dist = min_dist; c.max_dist = max_dist; c.min_angle_deg = min_angle_deg;
     c.min_frames = min_frames;
 }
@@ -227,7 +225,8 @@ static int triangulate_staged(b200vo_ctx* ctx, const double K[9], double min_dis
     VO_CUDA(ctx, cudaSetDevice(ctx->device));
     VO_CUDA(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
     TriBatchArgs b{};
-    vo_tri_common(b.common, K, min_dist, max_dist, min_baseline_angle_deg, min_baseline_frames);
+    vo_tri_common(b.common, min_dist, max_dist, min_baseline_angle_deg, min_baseline_frames);
+    VO_TRY(vo_intrinsics_uniform(ctx, K, VO_BOOT_EMAT_THR, batch, &b.intr));   // one K for every sequence
     b.cap = cap; b.pose_cap = pose_cap;
     const size_t nc = (size_t)batch * cap;
     const size_t b_k = vo_align(nc * 8, 256), b_fp = vo_align(nc * 4, 256), b_ps = vo_align((size_t)batch * pose_cap * 96, 256);
@@ -401,8 +400,9 @@ recover_cheirality_kernel(RecArgs a)
         }
         const float* p1 = a.p1 + 2 * po;
         const float* p2 = a.p2 + 2 * po;
-        const double x1 = ((double)p1[2 * i] - a.cx) / a.fx, y1 = ((double)p1[2 * i + 1] - a.cy) / a.fy;
-        const double x2 = ((double)p2[2 * i] - a.cx) / a.fx, y2 = ((double)p2[2 * i + 1] - a.cy) / a.fy;
+        const VoIntrinsics& c = a.intr[s];
+        const double x1 = ((double)p1[2 * i] - c.cx) / c.fx, y1 = ((double)p1[2 * i + 1] - c.cy) / c.fy;
+        const double x2 = ((double)p2[2 * i] - c.cx) / c.fx, y2 = ((double)p2[2 * i + 1] - c.cy) / c.fy;
         double A[16] = {-1, 0, x1, 0, 0, -1, y1, 0, 0, 0, 0, 0, 0, 0, 0, 0}, W[4], U[16], Vt[16], At[16];
 #pragma unroll
         for (int k = 0; k < 4; ++k) { A[8 + k] = x2 * P[8 + k] - P[k]; A[12 + k] = y2 * P[8 + k] - P[4 + k]; }
@@ -452,7 +452,8 @@ extern "C" int b200vo_recover_pose(b200vo_ctx* ctx, const double E[9], const flo
     VO_CUDA(ctx, cudaSetDevice(ctx->device));
     VO_CUDA(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
     RecArgs a{};
-    a.fx = K[0]; a.fy = K[4]; a.cx = K[2]; a.cy = K[5]; a.dist = distance_thresh; a.cap = n;
+    VO_TRY(vo_intrinsics_uniform(ctx, K, VO_BOOT_EMAT_THR, 1, &a.intr));   // the batch of one
+    a.dist = distance_thresh; a.cap = n;
     const int nn = n > 0 ? n : 1;
     const size_t b_p = vo_align((size_t)nn * 8, 256), b_m = vo_align((size_t)4 * nn, 256), b_small = 512;
     VO_TRY(vo_reserve(ctx, ctx->d_scratch[7], 2 * b_p + b_small + b_m + b_small));

@@ -5,7 +5,7 @@
 
 // one sequence's view of the triangulation kernels, built on the device by tri_sequence
 struct TriArgs {
-    double K[9], Ki[9];
+    const double* K; const double* Ki;   // the sequence's K and its inverse (its VoIntrinsics row)
     double cur[12];            // R_CW | t_CW of the current frame (as the reference stores them)
     double min_dist, max_dist, min_angle_deg;
     int min_frames, n, n_poses;
@@ -19,7 +19,8 @@ struct TriArgs {
 
 // batched forms: blockIdx.y (or blockIdx.x for the compaction) = sequence, ragged counts per sequence
 struct TriBatchArgs {
-    TriArgs common;            // K, Ki, gates (the per-sequence fields are filled in by the kernels)
+    TriArgs common;            // the gates (the per-sequence fields are filled in by the kernels)
+    const VoIntrinsics* intr;  // [batch] camera of each sequence
     int cap, pose_cap;
     const int* n;              // [batch] candidates per sequence
     const int* n_poses;        // [batch]
@@ -29,8 +30,8 @@ struct TriBatchArgs {
     uint8_t* keep; float* lm_slot; float* out_lm; float* out_kp; int* n_new; int* flags;   // [batch]...
 };
 
-// K, its inverse and the reference's gates (main.py:21-25) into the shared part of the argument block
-void vo_tri_common(TriArgs& c, const double K[9], double min_dist, double max_dist, double min_angle_deg, int min_frames);
+// the reference's gates (main.py:21-25) into the shared part of the argument block
+void vo_tri_common(TriArgs& c, double min_dist, double max_dist, double min_angle_deg, int min_frames);
 // triangulate_batch_kernel + triangulate_compact_batch_kernel on `stream`; every pointer of `b` is device memory
 int vo_triangulate_batch_launch(b200vo_ctx* ctx, const TriBatchArgs& b, int batch, cudaStream_t stream);
 // min_distance_batch_kernel on `stream` (valid rows >= n[s] are left as they are)
@@ -42,7 +43,8 @@ struct RecArgs {
     const double* E;           // [batch][9]
     const int* valid;          // nullptr or valid[valid_stride * s] != 0: decompose E of sequence s (others keep zero poses)
     int valid_stride;
-    double fx, fy, cx, cy, dist;
+    const VoIntrinsics* intr;  // [batch] camera of each sequence
+    double dist;
     int cap;
     const int* n;              // [batch]
     const float* p1; const float* p2;

@@ -246,7 +246,8 @@ extern "C" int b200vo_loop_create(b200vo_ctx* ctx, int batch, const b200vo_loop_
     d.n_cand_b = cnt + CNT_CAND_B * nb; d.tri_n = cnt + CNT_TRI * nb; d.n_new = cnt + CNT_NEW * nb; d.n_corner = cnt + CNT_CORNER * nb;
     d.c_obj = B->c_obj; d.c_img = B->c_img; d.c_n = B->c_n; d.inliers = B->inliers;
     TriBatchArgs& t = lp->tri;
-    vo_tri_common(t.common, bc.K, cfg->min_dist_landmarks, cfg->max_dist_landmarks, cfg->min_baseline_angle_deg, cfg->min_baseline_frames);
+    vo_tri_common(t.common, cfg->min_dist_landmarks, cfg->max_dist_landmarks, cfg->min_baseline_angle_deg, cfg->min_baseline_frames);
+    t.intr = B->intr;
     t.cap = C; t.pose_cap = P;
     t.n = d.tri_n; t.n_poses = d.n_poses; t.cur = d.cur_pose;
     t.first_keys = d.fkeys_b; t.keys = d.keys_b; t.first_pose = d.fpose_b; t.poses = d.poses;
@@ -402,6 +403,11 @@ extern "C" int b200vo_loop_load(b200vo_loop* lp, int seq, const uint8_t* frame, 
     for (int i = 0; i < 6; ++i) VO_CUDA(ctx, cudaMemcpyAsync(dst[i] + seq, v + i, 4, cudaMemcpyHostToDevice, st));
     VO_CUDA(ctx, cudaStreamSynchronize(st));
     return 0;
+}
+
+extern "C" int b200vo_loop_set_intrinsics(b200vo_loop* lp, int n_seq, const int32_t* seqs, const double* K)
+{
+    return lp ? batch_set_intrinsics(lp->B, n_seq, seqs, K) : B200VO_E_BADARG;
 }
 
 extern "C" int b200vo_loop_read_state(b200vo_loop* lp, int seq, float* lm, float* lm_kp, int32_t* n_lm, float* keys, float* first_keys,
@@ -595,7 +601,7 @@ extern "C" int b200vo_loop_bootstrap(b200vo_loop* lp, int n_seq, const int32_t* 
     const size_t nc = ns * cap, sq = std::max(sum_q, 1);
     const size_t sizes[] = {ns * BT_KINDS * 4, sq * 8, sq * 8, sq, nc * 8, nc * 8, ns * 4, ns * 72, nc, ns * 16, ns * 4,
                             nc * 8, nc * 8, ns * 4, nc * 4, ns * 384, ns * 16, ns * 96, ns * 8, ns * 96, ns * 4, ns * 4, ns * 96,
-                            nc, nc * 12, nc * 12, nc * 8, ns * 4, ns * 4, ns * 16, ns * sb};
+                            nc, nc * 12, nc * 12, nc * 8, ns * 4, ns * 4, ns * 16, ns * sb, ns * sizeof(VoIntrinsics)};
     size_t total = 0;
     for (size_t x : sizes) total += vo_align(x, 256);
     VO_TRY(vo_reserve(ctx, lp->boot_ws, total));
@@ -625,6 +631,12 @@ extern "C" int b200vo_loop_bootstrap(b200vo_loop* lp, int n_seq, const int32_t* 
     t.n_new = (int*)take(); t.flags = (int*)take();
     b.res = (int*)take();
     uint8_t* slab = (uint8_t*)take();
+    // the camera of each listed sequence, in list order (the bootstrap's kernels take the sequence from the grid)
+    VoIntrinsics* intr = (VoIntrinsics*)take();
+    std::vector<VoIntrinsics> h_intr(ns);
+    for (int k = 0; k < n_seq; ++k) h_intr[k] = B->intr_host[seqs[k]];
+    VO_CUDA(ctx, cudaMemcpyAsync(intr, h_intr.data(), ns * sizeof(VoIntrinsics), cudaMemcpyHostToDevice, st));
+    t.intr = intr;
     b.keep = t.keep; b.new_lm = t.out_lm; b.new_kp = t.out_kp; b.n_new = t.n_new;
     b.slab = slab; b.slab_bytes = sb; b.cur_slab = (uint8_t*)B->slabs[B->cur].p;
     VO_CUDA(ctx, cudaMemcpyAsync(d_tab, tab.data(), ns * BT_KINDS * 4, cudaMemcpyHostToDevice, st));
@@ -651,14 +663,13 @@ extern "C" int b200vo_loop_bootstrap(b200vo_loop* lp, int n_seq, const int32_t* 
     }
     boot_match_kernel<<<n_seq, LOOP_T, 0, st>>>(b);
     ctx->launches++;
-    // findEssentialMat(RANSAC, prob 0.99, threshold 1.0, maxIters 1000) at :308
-    const double* K = lp->cfg.batch.K;
-    VO_TRY(vo_emat_batch(ctx, b.pts0, b.pts1, cap, b.n_match, cap, n_seq, K, 0.99, 1.0, 1000, E, emask, eres, eflags));
+    // findEssentialMat(RANSAC, prob 0.99, threshold 1.0 = VO_BOOT_EMAT_THR, maxIters 1000) at :308
+    VO_TRY(vo_emat_batch(ctx, b.pts0, b.pts1, cap, b.n_match, cap, n_seq, intr, 0.99, 1000, E, emask, eres, eflags));
     boot_inliers_kernel<<<n_seq, LOOP_T, 0, st>>>(b);
     ctx->launches++;
     // recoverPose(E, inliers, K) with distanceThresh 50 (:315)
     ra.E = E; ra.valid = eres; ra.valid_stride = 4;
-    ra.fx = K[0]; ra.fy = K[4]; ra.cx = K[2]; ra.cy = K[5]; ra.dist = 50.0;
+    ra.intr = intr; ra.dist = 50.0;
     ra.cap = cap; ra.n = b.n_inl; ra.p1 = b.inl0; ra.p2 = b.inl1;
     VO_TRY(vo_recover_pose_batch_launch(ctx, ra, n_seq, cap, st));
     boot_pose_kernel<<<(n_seq + 127) / 128, 128, 0, st>>>(b);

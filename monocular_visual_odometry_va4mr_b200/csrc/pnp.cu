@@ -18,22 +18,27 @@
 
 using namespace vo;
 
+// One of the four camera doubles (fx, fy, cx, cy) of a sequence, read where it is used: the loads are not merged or hoisted,
+// so no register holds the camera across the solvers' long live ranges (the fused kernel is at its register limit)
+__device__ __forceinline__ double cam_at(const double* cam, int k) { return ((const volatile double*)cam)[k]; }
+
 // ------------------------------------------------------------------------------------------
 // 2. minimal solver: one thread per hypothesis
 // ------------------------------------------------------------------------------------------
 // One hypothesis: P3P on the first 3 points of the sample, the 4th picks the candidate.  Writes R|t (re-expanded
 // from rvec, as PnPRansacCallback stores its model) to h[12] and rvec to hr[3]; returns 0 when there is no model.
-__device__ inline int pnp_solve_one(const PnpArgs& a, const float* obj, const float* img, const int* smp, double* h, double* hr)
+// cam = the sequence's fx, fy, cx, cy.
+__device__ inline int pnp_solve_one(const double* cam, const float* obj, const float* img, const int* smp, double* h, double* hr)
 {
     double X[12], xn[8], uv[8];
-    const double ifx = 1. / a.fx, ify = 1. / a.fy;
+    const double ifx = 1. / cam_at(cam, 0), ify = 1. / cam_at(cam, 1);
     for (int k = 0; k < 4; ++k) {
         const int s = smp[k];
         X[3 * k] = obj[3 * s]; X[3 * k + 1] = obj[3 * s + 1]; X[3 * k + 2] = obj[3 * s + 2];
         uv[2 * k] = img[2 * s]; uv[2 * k + 1] = img[2 * s + 1];
         // cv2 normalises with undistortPoints on CV_32F input: double arithmetic, float32 result
-        xn[2 * k] = (double)(float)((uv[2 * k] - a.cx) * ifx);
-        xn[2 * k + 1] = (double)(float)((uv[2 * k + 1] - a.cy) * ify);
+        xn[2 * k] = (double)(float)((uv[2 * k] - cam_at(cam, 2)) * ifx);
+        xn[2 * k + 1] = (double)(float)((uv[2 * k + 1] - cam_at(cam, 3)) * ify);
     }
     double R[4][9], t[4][3];
     const int ns = p3p(X, xn, R, t);
@@ -43,7 +48,7 @@ __device__ inline int pnp_solve_one(const PnpArgs& a, const float* obj, const fl
         double e = 0;
         for (int k = 0; k < 4; ++k) {
             double u, v;
-            project_pt(R[s], t[s], a.fx, a.fy, a.cx, a.cy, X[3 * k], X[3 * k + 1], X[3 * k + 2], u, v);
+            project_pt(R[s], t[s], cam_at(cam, 0), cam_at(cam, 1), cam_at(cam, 2), cam_at(cam, 3), X[3 * k], X[3 * k + 1], X[3 * k + 2], u, v);
             const double dx = uv[2 * k] - u, dy = uv[2 * k + 1] - v;
             e += dx * dx + dy * dy;
         }
@@ -74,7 +79,7 @@ pnp_solve_kernel(PnpArgs a)
     const int* smp = a.samples + hidx * 4;
     const int N = a.n[b];
     if (smp[0] < 0 || N < 4) return;
-    a.hyp_ok[hidx] = pnp_solve_one(a, a.obj + (size_t)b * a.cap * 3, a.img + (size_t)b * a.cap * 2, smp, a.hyp + hidx * 12,
+    a.hyp_ok[hidx] = pnp_solve_one(&a.intr[b].fx, a.obj + (size_t)b * a.cap * 3, a.img + (size_t)b * a.cap * 2, smp, a.hyp + hidx * 12,
                                    a.hyp_rvec + hidx * 3);
 }
 
@@ -154,9 +159,11 @@ pnp_score_kernel(PnpArgs a)
         iu = m[0]; iv = m[1];
     }
     const int lane = threadIdx.x & 31;
+    const VoIntrinsics& cam = a.intr[b];
+    const double fx = cam.fx, fy = cam.fy, cx = cam.cx, cy = cam.cy;
     for (int h = 0; h < nh; ++h) {
         if (!s_ok[h]) continue;   // block-uniform
-        const bool in = live && pnp_is_inlier(s_h + h * 12, a.fx, a.fy, a.cx, a.cy, X, Y, Z, iu, iv, a.thr_sq);
+        const bool in = live && pnp_is_inlier(s_h + h * 12, fx, fy, cx, cy, X, Y, Z, iu, iv, a.thr_sq);
         const unsigned m = __ballot_sync(0xffffffffu, in);
         if (lane == 0 && m) atomicAdd(a.counts + hbase + h, __popc(m));
     }
@@ -211,7 +218,7 @@ pnp_select_kernel(PnpArgs a)
             else {
                 const float* o = a.obj + ((size_t)b * a.cap + i) * 3;
                 const float* m = a.img + ((size_t)b * a.cap + i) * 2;
-                in = pnp_is_inlier(s_h, a.fx, a.fy, a.cx, a.cy, o[0], o[1], o[2], m[0], m[1], a.thr_sq);
+                in = pnp_is_inlier(s_h, a.intr[b].fx, a.intr[b].fy, a.intr[b].cx, a.intr[b].cy, o[0], o[1], o[2], m[0], m[1], a.thr_sq);
             }
         }
         mask[i] = in ? 1 : 0;
@@ -430,12 +437,13 @@ __device__ inline void epnp_gauss_newton(const double* L, const double* rho, dou
 
 // The refit, executed by one CTA of EPNP_T threads (every thread must call it; S is the CTA's scratch):
 // obj/img are this sequence's correspondences, inl[0..M) the inlier indices, pose_out receives rvec|tvec
-// (left untouched when the result is not finite -- the caller has put the RANSAC model there).
-__device__ inline void epnp_block(const PnpArgs& a, EpnpShared& S, const float* obj, const float* img, const int* inl, int M, double* pose_out, int b)
+// (left untouched when the result is not finite -- the caller has put the RANSAC model there); cam = fx, fy, cx, cy.
+__device__ inline void epnp_block(const PnpArgs& a, const double* cam, EpnpShared& S, const float* obj, const float* img, const int* inl, int M,
+                                  double* pose_out, int b)
 {
     const int tid = threadIdx.x;
     const double n = (double)M;
-    const double ifx = 1. / a.fx, ify = 1. / a.fy;
+    const double ifx = 1. / cam_at(cam, 0), ify = 1. / cam_at(cam, 1);
     // tournament partner table (built here, consumed after several barriers)
     for (int k = tid; k < 66; k += EPNP_T) {
         const int rnd = k / 6, pr = k - rnd * 6;
@@ -493,9 +501,10 @@ __device__ inline void epnp_block(const PnpArgs& a, EpnpShared& S, const float* 
         for (int j = 0; j < 3; ++j) al[1 + j] = ci[3 * j] * dx + ci[3 * j + 1] * dy + ci[3 * j + 2] * dz;
         al[0] = 1.0 - al[1] - al[2] - al[3];
         // undistortPoints (float64) then back to pixels, as cv2's EPnP front end does
-        const double u = (((double)img[2 * id] - a.cx) * ifx) * a.fx + a.cx;
-        const double v = (((double)img[2 * id + 1] - a.cy) * ify) * a.fy + a.cy;
-        const double du = a.cx - u, dv = a.cy - v, dd = du * du + dv * dv;
+        const double fx = cam_at(cam, 0), fy = cam_at(cam, 1), cx = cam_at(cam, 2), cy = cam_at(cam, 3);
+        const double u = (((double)img[2 * id] - cx) * ifx) * fx + cx;
+        const double v = (((double)img[2 * id + 1] - cy) * ify) * fy + cy;
+        const double du = cx - u, dv = cy - v, dd = du * du + dv * dv;
 #define EPNP_PAIR(slot, j, l) { const double aa = al[j] * al[l]; acc[4 * (slot)] += aa; acc[4 * (slot) + 1] += aa * du; \
                                 acc[4 * (slot) + 2] += aa * dv; acc[4 * (slot) + 3] += aa * dd; }
 #define EPNP_MOM(slot, j) { acc[20 + 3 * (slot)] += al[j] * X; acc[20 + 3 * (slot) + 1] += al[j] * Y; acc[20 + 3 * (slot) + 2] += al[j] * Z; \
@@ -539,11 +548,11 @@ __device__ inline void epnp_block(const PnpArgs& a, EpnpShared& S, const float* 
         const int q = jb * 4 - jb * (jb - 1) / 2 + (lb - jb);                    // index of (jb <= lb) in the upper triangle
         const double A = S.out[4 * q], B = S.out[4 * q + 1], Cc = S.out[4 * q + 2], D = S.out[4 * q + 3];
         double v;
-        if (r == 0 && c == 0) v = a.fx * a.fx * A;
-        else if (r == 1 && c == 1) v = a.fy * a.fy * A;
+        if (r == 0 && c == 0) v = cam_at(cam, 0) * cam_at(cam, 0) * A;
+        else if (r == 1 && c == 1) v = cam_at(cam, 1) * cam_at(cam, 1) * A;
         else if (r == 2 && c == 2) v = D;
-        else if ((r == 0 && c == 2) || (r == 2 && c == 0)) v = a.fx * B;
-        else if ((r == 1 && c == 2) || (r == 2 && c == 1)) v = a.fy * Cc;
+        else if ((r == 0 && c == 2) || (r == 2 && c == 0)) v = cam_at(cam, 0) * B;
+        else if ((r == 1 && c == 2) || (r == 2 && c == 1)) v = cam_at(cam, 1) * Cc;
         else v = 0.0;
         S.jac[0][tid] = v;
     }
@@ -624,8 +633,9 @@ __device__ inline void epnp_block(const PnpArgs& a, EpnpShared& S, const float* 
         const int id = inl[k];
         const float* o = obj + 3 * id;
         const double X = o[0], Y = o[1], Z = o[2];
-        const double u = (((double)img[2 * id] - a.cx) * ifx) * a.fx + a.cx;
-        const double v = (((double)img[2 * id + 1] - a.cy) * ify) * a.fy + a.cy;
+        const double fx = cam_at(cam, 0), fy = cam_at(cam, 1), cx = cam_at(cam, 2), cy = cam_at(cam, 3);
+        const double u = (((double)img[2 * id] - cx) * ifx) * fx + cx;
+        const double v = (((double)img[2 * id + 1] - cy) * ify) * fy + cy;
 #pragma unroll
         for (int c = 0; c < 3; ++c) {
             const double* R = S.Rs[c];
@@ -633,7 +643,7 @@ __device__ inline void epnp_block(const PnpArgs& a, EpnpShared& S, const float* 
             const double Xc = R[0] * X + R[1] * Y + R[2] * Z + t[0];
             const double Yc = R[3] * X + R[4] * Y + R[5] * Z + t[1];
             const double iZ = 1.0 / (R[6] * X + R[7] * Y + R[8] * Z + t[2]);
-            const double ue = a.cx + a.fx * Xc * iZ, ve = a.cy + a.fy * Yc * iZ;
+            const double ue = cx + fx * Xc * iZ, ve = cy + fy * Yc * iZ;
             const double du = u - ue, dv = v - ve;
             acc[c] += sqrt(du * du + dv * dv);
         }
@@ -667,7 +677,7 @@ pnp_epnp_kernel(PnpArgs a)
     const int N = a.n[b];
     const int M = a.n_inliers[b];
     if (N == 4 || M < 4) return;   // N == 4: cv2 returns the direct P3P solve
-    epnp_block(a, S, a.obj + (size_t)b * a.cap * 3, a.img + (size_t)b * a.cap * 2, a.inliers + (size_t)b * a.cap, M,
+    epnp_block(a, &a.intr[b].fx, S, a.obj + (size_t)b * a.cap * 3, a.img + (size_t)b * a.cap * 2, a.inliers + (size_t)b * a.cap, M,
                a.pose + (size_t)b * 6, b);
 }
 
@@ -692,6 +702,7 @@ struct PoseFusedShared {
     int ok[FUSED_CHUNK], cnt[FUSED_CHUNK];
     int smp[FUSED_CHUNK * 4];
     int mod[FUSED_WIN];
+    double cam[4];      // the sequence's fx, fy, cx, cy, loaded once per CTA
     int warp_n[8];
     int base, N, niters, max_good, win, it0, pos, nh;
 };
@@ -773,6 +784,7 @@ pnp_fused_kernel(PnpArgs a, PoseBatchIO io)
     // ---- 1. status == 1 landmarks, in order (what `matched_pts[tracked]` does in the reference, :282-284) ----
     // (written out rather than cta_compact: this kernel's register allocation is at its limit, <2> spills)
     if (tid == 0) F.base = 0;
+    const double cam_r = tid < 4 ? (&a.intr[b].fx)[tid] : 0.0;   // issued now, stored after the compaction (hides the latency)
     __syncthreads();
     if (io.lm_status) {
         const int n = min(max(io.n_lm[b], 0), a.cap);   // a count beyond the slot capacity must not reach the neighbour's arrays
@@ -806,6 +818,7 @@ pnp_fused_kernel(PnpArgs a, PoseBatchIO io)
         F.niters = N == 4 ? 1 : (N > 4 ? (a.iters > 1 ? a.iters : 1) : 0);
         F.max_good = 0; F.win = -1; F.it0 = 0; F.pos = 0;
     }
+    if (tid < 4) F.cam[tid] = cam_r;
     __syncthreads();
 
     phase_stamp(a, b, 1);   // compaction done
@@ -824,7 +837,7 @@ pnp_fused_kernel(PnpArgs a, PoseBatchIO io)
         if ((tid & 7) == 0) {
             const int h = tid >> 3;
             int okh = 0;
-            if (h < nh && F.smp[4 * h] >= 0) okh = pnp_solve_one(a, obj, img, F.smp + 4 * h, F.h + 12 * h, F.rv + 3 * h);
+            if (h < nh && F.smp[4 * h] >= 0) okh = pnp_solve_one(F.cam, obj, img, F.smp + 4 * h, F.h + 12 * h, F.rv + 3 * h);
             F.ok[h] = okh;
         }
         __syncthreads();
@@ -835,6 +848,7 @@ pnp_fused_kernel(PnpArgs a, PoseBatchIO io)
         for (int h_lo = 0; h_lo < nh; h_lo += FUSED_SUB) {
             const int h_hi = min(h_lo + FUSED_SUB, nh);
             if (N > 4) {
+                const double fx = F.cam[0], fy = F.cam[1], cx = F.cam[2], cy = F.cam[3];   // registers for the scoring loop only
                 for (int base = 0; base < N; base += FUSED_T) {
                     const int i = base + tid;
                     const bool live = i < N;
@@ -845,7 +859,7 @@ pnp_fused_kernel(PnpArgs a, PoseBatchIO io)
                     // points x 32 hypotheses -- with eight warps on the SM the phase is bound by issue latency, not by the FP64 pipe)
                     for (int h = h_lo; h < h_hi; ++h) {
                         if (!F.ok[h]) continue;   // block-uniform
-                        const bool in = live && pnp_is_inlier(F.h + h * 12, a.fx, a.fy, a.cx, a.cy, X, Y, Z, iu, iv, a.thr_sq);
+                        const bool in = live && pnp_is_inlier(F.h + h * 12, fx, fy, cx, cy, X, Y, Z, iu, iv, a.thr_sq);
                         const unsigned m = __ballot_sync(0xffffffffu, in);
                         if (lane == 0 && m) atomicAdd(&F.cnt[h], __popc(m));
                     }
@@ -890,7 +904,7 @@ pnp_fused_kernel(PnpArgs a, PoseBatchIO io)
         for (int base = 0; base < a.cap; base += FUSED_T) {
             const int i = base + tid;
             bool in = false;
-            if (i < N) in = N == 4 ? true : pnp_is_inlier(F.win_h, a.fx, a.fy, a.cx, a.cy, obj[3 * i], obj[3 * i + 1], obj[3 * i + 2], img[2 * i], img[2 * i + 1], a.thr_sq);
+            if (i < N) in = N == 4 ? true : pnp_is_inlier(F.win_h, cam_at(F.cam, 0), cam_at(F.cam, 1), cam_at(F.cam, 2), cam_at(F.cam, 3), obj[3 * i], obj[3 * i + 1], obj[3 * i + 2], img[2 * i], img[2 * i + 1], a.thr_sq);
             const unsigned bm = __ballot_sync(0xffffffffu, in);
             if (lane == 0) F.warp_n[warp] = __popc(bm);
             __syncthreads();
@@ -917,7 +931,7 @@ pnp_fused_kernel(PnpArgs a, PoseBatchIO io)
         __syncthreads();
         phase_stamp(a, b, 3);   // winner mask + inlier list done
         // ---- 4. EPnP refit on the inliers (N == 4: cv2 returns the direct P3P solve) ----
-        if (N != 4 && M >= 4) epnp_block(a, S, obj, img, inl, M, pose, b);
+        if (N != 4 && M >= 4) epnp_block(a, F.cam, S, obj, img, inl, M, pose, b);
     }
     phase_stamp(a, b, 8);   // EPnP done
     // ---- 5. inlier mask over the ORIGINAL landmark slots (:346) ----

@@ -5,13 +5,14 @@
 #include <cstddef>
 
 struct b200vo_ctx;
+struct VoIntrinsics;
 
 struct PnpArgs {
     int batch, cap, iters;
     const float* obj;       // [batch][cap][3]
     const float* img;       // [batch][cap][2]
     const int* n;           // [batch] live correspondences per sequence
-    double fx, fy, cx, cy;
+    const VoIntrinsics* intr;   // [batch] camera of each sequence (fx, fy, cx, cy)
     float thr_sq;           // (float)(reprojectionError^2)
     double conf;
     const uint32_t* rng_raw;  // raw cv::RNG((uint64)-1) outputs

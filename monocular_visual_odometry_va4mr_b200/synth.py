@@ -124,12 +124,13 @@ class Corridor:
 
 
 def render_sequence(shape: str = "kitti", n_frames: int = 3, seed: int = 0, start: int = 0,
-                    width: int | None = None, height: int | None = None):
-    """Frames, depths and poses for a dataset-shaped sequence.
+                    width: int | None = None, height: int | None = None, K: np.ndarray | None = None):
+    """Frames, depths and poses for a dataset-shaped sequence, seen by the dataset's camera or by ``K`` (3, 3).
 
     Returns dict(K, frames [n,H,W] u8, depth [n,H,W] f64, R_cw [n,3,3], c [n,3]).
     """
-    K, w, h, step, _ = SHAPES[shape]
+    K0, w, h, step, _ = SHAPES[shape]
+    K = K0 if K is None else np.asarray(K, np.float64).reshape(3, 3)
     w = width or w
     h = height or h
     scene = Corridor(seed)
