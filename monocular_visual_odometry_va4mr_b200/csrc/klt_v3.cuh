@@ -5,7 +5,8 @@
 //     with funnel shifts: with lanes 0-15 on the left runs and lanes 16-31 on the right runs each half-warp
 //     touches 15 distinct slots, so the window reads are conflict-free;
 //   * the bilinear interpolation I00*w00 + I01*w01 (+ next row) is two dp2a (16-bit weights x 8-bit pixels)
-//     instead of four IMAD; the Scharr derivative of the previous image is 5 dp4a per pixel on the staged patch;
+//     instead of four IMAD; the template gradients are Scharr of the unrounded bilinear image when the window's tap
+//     grid lies inside the image (template_interior), otherwise 5 dp4a per tap on the staged patch, interpolated;
 //   * the window of the NEXT image is staged in shared memory per level by 8-byte cp.async (window + 4 px
 //     margin, restaged only if the point leaves it), so iterations never touch L1/L2;
 //   * the template gradients live in registers; sum(Iwin*dI) is folded into two constants, so an iteration
@@ -16,8 +17,9 @@
 //   * iteration loop: the staged-window test and the image-range test are ONE unsigned compare per axis
 //     against bounds fixed at staging time; plain F2I.FLOOR instead of the guarded cvFloor (positions are
 //     finite inside the loop, the guard stays at the level entry); the two exact 64-bit warp sums take a
-//     single-REDUX fast path whenever no lane partial can overflow int32 (a vote decides; the hi/lo split
-//     path is kept for the rest); packed weights by one IMAD each.
+//     single-REDUX fast path when a per-level bound rules out an int32 overflow (ITER_SUM_FAST_MAX; the hi/lo
+//     split path is kept for the rest); packed weights by one IMAD each;
+//   * Iwin and the final error pass are skipped when the point set has no error output.
 #pragma once
 #include <type_traits>
 
@@ -78,6 +80,10 @@ struct KV3 {
     static constexpr int B_IWIN = ((IS * WH * 2 + 15) / 16) * 16;
     static constexpr int PER_WARP = 2 * B_PATCH + B_J + 2 * B_DER + B_IWIN;   // two patch buffers (prefetch)
     static constexpr int MIN_CTAS = ((227 * 1024) / (KLT_WARPS * PER_WARP + 64 + 1024) * KLT_WARPS >= 32 ? 32 : 24) / KLT_WARPS;
+    // An iteration's lane partial is sum (IvJ - Iwin) * dIx over the lane's 8 * NROUND pixels, with IvJ and Iwin in
+    // [0, 8160]; by Cauchy-Schwarz |partial| <= 8160 * sqrt(8 * NROUND * sum dIx^2).  A lane sum of dIx^2 (and of
+    // dIy^2) up to this bound keeps every partial of the level below 2^26: the single-REDUX sums are exact.
+    static constexpr int ITER_SUM_FAST_MAX = (int)(((1ll << 52) - 1) / (8160ll * 8160ll * (8 * NROUND)));
 };
 
 __device__ __forceinline__ unsigned long long global_timer_ns()
@@ -141,16 +147,79 @@ __device__ __forceinline__ void interp_run8_64(uint32_t img_s, int off, int sh8,
 }
 
 // Exact sums of two int32 values over the warp, as float32 (== __ll2float_rn of the 64-bit sums).  A lane partial
-// below 2^26 in magnitude cannot overflow the 32-lane int32 sum: one REDUX each; otherwise the hi/lo split path.
-__device__ __forceinline__ void warp_sum2_f32(int v1, int v2, float& f1, float& f2)
+// below 2^26 in magnitude cannot overflow the 32-lane int32 sum: one REDUX each; otherwise (wide) the hi/lo split
+// path.  Both give the same float whenever the single REDUX is exact.
+__device__ __forceinline__ void warp_sum2_f32(int v1, int v2, bool wide, float& f1, float& f2)
 {
-    const int m = max(abs(v1), abs(v2));
-    if (__any_sync(0xffffffffu, m >= (1 << 26))) {
+    if (wide) {
         f1 = __ll2float_rn(warp_sum_i64(v1));
         f2 = __ll2float_rn(warp_sum_i64(v2));
     } else {
         f1 = __int2float_rn(__reduce_add_sync(0xffffffffu, v1));
         f2 = __int2float_rn(__reduce_add_sync(0xffffffffu, v2));
+    }
+}
+__device__ __forceinline__ void warp_sum2_f32(int v1, int v2, float& f1, float& f2)
+{
+    warp_sum2_f32(v1, v2, __any_sync(0xffffffffu, max(abs(v1), abs(v2)) >= (1 << 26)), f1, f2);
+}
+
+// Template derivatives of a window whose whole tap grid lies inside the image, for the split layout (lane = window
+// row ty = lane & 15, columns tx .. tx+7).  Scharr is linear, so the bilinear blend of Scharr taps equals Scharr of
+// the unrounded bilinear image U(u, v) = iw00 p(u,v) + iw01 p(u+1,v) + iw10 p(u,v+1) + iw11 p(u+1,v+1), exactly in
+// int32 (|Scharr(U)| <= 16 * 255 * (2^14 + 2) < 2^31).  With no tap zeroed at the image border this is the value
+// the tap grid gives, bit for bit.  The lane computes U on rows ty-1 and ty for columns tx-1 .. tx+8 and takes row
+// ty+1 from the next lane (the last lane of each half computes row WH for it).  The dp2a chains carry the +2^8 of
+// the rounding of Iv; the Scharr kernels sum to zero, so it cancels in the derivatives.
+template <bool HI>
+__device__ __forceinline__ void patch_row_pairs10(uint32_t addr8, int sh8, uint32_t* w)
+{
+    const uint2 A = lds_u64(addr8), B = lds_u64(addr8 + 8);
+    uint32_t t0, t1, t2, t3;
+    if (HI) { const uint2 Cc = lds_u64(addr8 + 16); t0 = A.y; t1 = B.x; t2 = B.y; t3 = Cc.x; }
+    else { t0 = A.x; t1 = A.y; t2 = B.x; t3 = B.y; }
+    const uint32_t a0 = __funnelshift_r(t0, t1, sh8), a1 = __funnelshift_r(t1, t2, sh8), a2 = __funnelshift_r(t2, t3, sh8);
+    w[0] = a0; w[1] = __funnelshift_r(a0, a1, 8); w[2] = a1; w[3] = __funnelshift_r(a1, a2, 8); w[4] = a2; w[5] = a2 >> 8;
+}
+// U (+2^8) of columns c = 0..9 from the pair words of the row (top) and the row below (bot)
+__device__ __forceinline__ void interp_row10(const uint32_t* top, const uint32_t* bot, uint32_t wt, uint32_t wb, int* U)
+{
+    const uint32_t R = 1u << (W_BITS - 5 - 1);
+#pragma unroll
+    for (int q = 0; q < 3; ++q) {
+        const int c = 4 * q;
+        U[c] = (int)dp2a_lo_u(wb, bot[2 * q], dp2a_lo_u(wt, top[2 * q], R));
+        U[c + 1] = (int)dp2a_lo_u(wb, bot[2 * q + 1], dp2a_lo_u(wt, top[2 * q + 1], R));
+        if (q < 2) {
+            U[c + 2] = (int)dp2a_hi_u(wb, bot[2 * q], dp2a_hi_u(wt, top[2 * q], R));
+            U[c + 3] = (int)dp2a_hi_u(wb, bot[2 * q + 1], dp2a_hi_u(wt, top[2 * q + 1], R));
+        }
+    }
+}
+template <int PS, bool HI>
+__device__ __forceinline__ void template_interior(uint32_t patch_s, int row_off, int sh8, uint32_t wt, uint32_t wb,
+                                                  int* gx, int* gy, int* Iv)
+{
+    // row_off: byte of pixel (tx-1, ty-1), rounded down to 8
+    uint32_t pa[6], pb[6], pc[6];
+    patch_row_pairs10<HI>(patch_s + row_off, sh8, pa);
+    patch_row_pairs10<HI>(patch_s + row_off + PS, sh8, pb);
+    patch_row_pairs10<HI>(patch_s + row_off + 2 * PS, sh8, pc);
+    int Um[10], U0[10];
+    interp_row10(pa, pb, wt, wb, Um);
+    interp_row10(pb, pc, wt, wb, U0);
+    int S[10], D[10];
+#pragma unroll
+    for (int c = 0; c < 10; ++c) {
+        const int Up = __shfl_down_sync(0xffffffffu, U0[c], 1, 16);
+        D[c] = Up - Um[c];
+        S[c] = (Up + Um[c]) * 3 + U0[c] * 10;
+    }
+#pragma unroll
+    for (int k = 0; k < 8; ++k) {
+        gx[k] = (S[k + 2] - S[k] + (1 << (W_BITS - 1))) >> W_BITS;
+        gy[k] = ((D[k] + D[k + 2]) * 3 + D[k + 1] * 10 + (1 << (W_BITS - 1))) >> W_BITS;
+        Iv[k] = (int)((uint32_t)U0[k + 1] >> (W_BITS - 5));
     }
 }
 
@@ -223,6 +292,7 @@ klt_kernel_v3(const KltArgs a)
     const uint8_t* next = a.next + (size_t)seq * a.next_stride;
     const size_t pidx = (size_t)seq * a.cap[seg] + pi;
     const float px0 = a.pts[seg][2 * pidx], py0 = a.pts[seg][2 * pidx + 1];
+    const bool want_err = a.err[seg] != nullptr;   // Iwin and the final error are only needed for this
     float outx = 0.f, outy = 0.f;
     int st = 1;
     float e = 0.f;
@@ -237,7 +307,7 @@ klt_kernel_v3(const KltArgs a)
         const int pitch = a.pitch[level];
         const uint8_t* I = prev + a.off[level];
         const uint8_t* J = next + a.off[level];
-        const float sc = (float)(1.0 / (double)(1 << level));
+        const float sc = __int_as_float((127 - level) << 23);   // exactly 2^-level
         float ppx = __fmul_rn(px0, sc), ppy = __fmul_rn(py0, sc);
         float nx, ny;
         if (level == a.levels - 1) { nx = ppx; ny = ppy; }
@@ -289,7 +359,7 @@ klt_kernel_v3(const KltArgs a)
         bool pf_next = false;
         if (level > 0) {
             const int nl = level - 1;
-            const float sc2 = (float)(1.0 / (double)(1 << nl));
+            const float sc2 = __int_as_float((127 - nl) << 23);
             const int qx = floor_to_int(__fsub_rn(__fmul_rn(px0, sc2), hwx)), qy = floor_to_int(__fsub_rn(__fmul_rn(py0, sc2), hwy));
             if (!(qx < -WW || qx >= a.w[nl] || qy < -WH || qy >= a.h[nl])) {
                 const uint8_t* n0 = prev + a.off[nl] + (long long)(qy - 1) * a.pitch[nl] + (qx - 1);
@@ -303,93 +373,107 @@ klt_kernel_v3(const KltArgs a)
         __syncwarp();
         // patch pixel (x, y), x in [-1, WW+1], y in [-1, WH+1], lives at byte (y+1)*PS + mis + 1 + x
 
-        // ---- Scharr on the tap grid: 5 dp4a per pixel, zero outside the image ----
-#pragma unroll
-        for (int r = 0; r < C::DROUND; ++r) {
-            const int t = r * 32 + lane;
-            if (t < C::DTASK) {
-                const int gy = t / C::DSEG, gx0 = (t - gy * C::DSEG) * 8;
-                const int off = gy * C::PS + mis + gx0;      // byte of pixel (gx0-1, gy-1)
-                const int sh8 = (off & 3) * 8;
-                int ix[8], iy[8];
-#pragma unroll
-                for (int k = 0; k < 8; ++k) { ix[k] = 0; iy[k] = 0; }
-#pragma unroll
-                for (int rr = 0; rr < 3; ++rr) {
-                    const uint32_t* w = reinterpret_cast<const uint32_t*>(patch + (off & ~3) + rr * C::PS);
-                    const uint32_t w0 = w[0], w1 = w[1], w2 = w[2], w3 = w[3];
-                    const uint32_t a0 = __funnelshift_r(w0, w1, sh8), a1 = __funnelshift_r(w1, w2, sh8), a2 = __funnelshift_r(w2, w3, sh8);
-                    uint32_t q[8];
-                    q[0] = a0; q[1] = __funnelshift_r(a0, a1, 8); q[2] = __funnelshift_r(a0, a1, 16); q[3] = __funnelshift_r(a0, a1, 24);
-                    q[4] = a1; q[5] = __funnelshift_r(a1, a2, 8); q[6] = __funnelshift_r(a1, a2, 16); q[7] = __funnelshift_r(a1, a2, 24);
-                    // q[k] = pixels (x-1, x, x+1, x+2) of row gy-1+rr for x = gx0+k
-                    const int cx = rr == 1 ? 0x000A00F6 : 0x000300FD;                  // (-10,0,10,0) / (-3,0,3,0)
-                    const int cy = rr == 0 ? 0x00FDF6FD : 0x00030A03;                  // (-3,-10,-3,0) / (3,10,3,0)
-#pragma unroll
-                    for (int k = 0; k < 8; ++k) {
-                        ix[k] = dp4a_us(q[k], cx, ix[k]);
-                        if (rr != 1) iy[k] = dp4a_us(q[k], cy, iy[k]);
-                    }
-                }
-                const int X0 = ipx + gx0, Y = ipy + gy;
-                const bool rowok = Y >= 0 && Y < lh;
-                if (!(rowok && X0 >= 0 && X0 + 7 < lw)) {
-#pragma unroll
-                    for (int k = 0; k < 8; ++k) {
-                        const bool ok = rowok && X0 + k >= 0 && X0 + k < lw;
-                        ix[k] = ok ? ix[k] : 0; iy[k] = ok ? iy[k] : 0;
-                    }
-                }
-                int4* dxp = reinterpret_cast<int4*>(derx + gy * C::DS + gx0);
-                int4* dyp = reinterpret_cast<int4*>(dery + gy * C::DS + gx0);
-                dxp[0] = make_int4(ix[0], ix[1], ix[2], ix[3]); dxp[1] = make_int4(ix[4], ix[5], ix[6], ix[7]);
-                dyp[0] = make_int4(iy[0], iy[1], iy[2], iy[3]); dyp[1] = make_int4(iy[4], iy[5], iy[6], iy[7]);
-            }
-        }
-        __syncwarp();
-
-        // ---- template: Iwin (smem), dIx/dIy (registers), normal matrix, sum(Iwin*dI) ----
+        // ---- template: dIx/dIy (registers), normal matrix, sum(Iwin*dI), Iwin (smem, only for the error) ----
         const uint32_t wt = (uint32_t)(iw01 * 65536 + iw00), wb = (uint32_t)iw11 * 65536u + (uint32_t)iw10;
         int gxr[C::NROUND][8], gyr[C::NROUND][8];
         int sA11 = 0, sA12 = 0, sA22 = 0, c1 = 0, c2 = 0;
-#pragma unroll
-        for (int r = 0; r < C::NROUND; ++r) {
-            const int off = (ty[r] + 1) * C::PS + mis + 1 + tx[r];
-            int Iv[8];
-            if (off & 4) interp_run8_64<C::PS, true>(patch_s, off, (off & 3) * 8, wt, wb, Iv);
-            else interp_run8_64<C::PS, false>(patch_s, off, (off & 3) * 8, wt, wb, Iv);
-            const int* d0 = derx + ty[r] * C::DS + tx[r];
-            const int* e0 = dery + ty[r] * C::DS + tx[r];
-            int dx0[9], dx1[9], dy0[9], dy1[9];
-            {
-                const int4 p0 = *reinterpret_cast<const int4*>(d0), p1 = *reinterpret_cast<const int4*>(d0 + 4);
-                const int4 q0 = *reinterpret_cast<const int4*>(d0 + C::DS), q1 = *reinterpret_cast<const int4*>(d0 + C::DS + 4);
-                dx0[0] = p0.x; dx0[1] = p0.y; dx0[2] = p0.z; dx0[3] = p0.w; dx0[4] = p1.x; dx0[5] = p1.y; dx0[6] = p1.z; dx0[7] = p1.w; dx0[8] = d0[8];
-                dx1[0] = q0.x; dx1[1] = q0.y; dx1[2] = q0.z; dx1[3] = q0.w; dx1[4] = q1.x; dx1[5] = q1.y; dx1[6] = q1.z; dx1[7] = q1.w; dx1[8] = d0[C::DS + 8];
-                const int4 r0 = *reinterpret_cast<const int4*>(e0), r1 = *reinterpret_cast<const int4*>(e0 + 4);
-                const int4 s0 = *reinterpret_cast<const int4*>(e0 + C::DS), s1 = *reinterpret_cast<const int4*>(e0 + C::DS + 4);
-                dy0[0] = r0.x; dy0[1] = r0.y; dy0[2] = r0.z; dy0[3] = r0.w; dy0[4] = r1.x; dy0[5] = r1.y; dy0[6] = r1.z; dy0[7] = r1.w; dy0[8] = e0[8];
-                dy1[0] = s0.x; dy1[1] = s0.y; dy1[2] = s0.z; dy1[3] = s0.w; dy1[4] = s1.x; dy1[5] = s1.y; dy1[6] = s1.z; dy1[7] = s1.w; dy1[8] = e0[C::DS + 8];
-            }
-            short iws[8];
+        auto accumulate = [&](int r, const int* ix, const int* iy, const int* Iv) {
 #pragma unroll
             for (int k = 0; k < 8; ++k) {
                 const bool livek = k < tl[r];
-                int ixv = (dx0[k] * iw00 + dx0[k + 1] * iw01 + dx1[k] * iw10 + dx1[k + 1] * iw11 + (1 << (W_BITS - 1))) >> W_BITS;
-                int iyv = (dy0[k] * iw00 + dy0[k + 1] * iw01 + dy1[k] * iw10 + dy1[k + 1] * iw11 + (1 << (W_BITS - 1))) >> W_BITS;
-                ixv = livek ? ixv : 0; iyv = livek ? iyv : 0;
+                const int ixv = livek ? ix[k] : 0, iyv = livek ? iy[k] : 0;
                 gxr[r][k] = ixv; gyr[r][k] = iyv;
-                iws[k] = (short)Iv[k];
                 sA11 += ixv * ixv; sA12 += ixv * iyv; sA22 += iyv * iyv;
                 c1 += Iv[k] * ixv; c2 += Iv[k] * iyv;
             }
-            if (tl[r] > 0) {
+            if (want_err && tl[r] > 0) {
                 uint4 pk;
-                pk.x = (uint16_t)iws[0] | ((uint32_t)(uint16_t)iws[1] << 16); pk.y = (uint16_t)iws[2] | ((uint32_t)(uint16_t)iws[3] << 16);
-                pk.z = (uint16_t)iws[4] | ((uint32_t)(uint16_t)iws[5] << 16); pk.w = (uint16_t)iws[6] | ((uint32_t)(uint16_t)iws[7] << 16);
+                pk.x = (uint16_t)Iv[0] | ((uint32_t)(uint16_t)Iv[1] << 16); pk.y = (uint16_t)Iv[2] | ((uint32_t)(uint16_t)Iv[3] << 16);
+                pk.z = (uint16_t)Iv[4] | ((uint32_t)(uint16_t)Iv[5] << 16); pk.w = (uint16_t)Iv[6] | ((uint32_t)(uint16_t)Iv[7] << 16);
                 *reinterpret_cast<uint4*>(Iwin + ty[r] * C::IS + tx[r]) = pk;
             }
+        };
+        // the whole tap grid (pixels ip + [0, WW] x [0, WH]) inside the image: no tap is zeroed
+        if (C::SPLIT && ipx >= 0 && ipx + WW < lw && ipy >= 0 && ipy + WH < lh) {
+            const int off = (lane & 15) * C::PS + mis + tx[0];   // byte of pixel (tx-1, row-1); off & 7 == mis
+            int ix[8], iy[8], Iv[8];
+            if (off & 4) template_interior<C::PS, true>(patch_s, off & ~7, (off & 3) * 8, wt, wb, ix, iy, Iv);
+            else template_interior<C::PS, false>(patch_s, off & ~7, (off & 3) * 8, wt, wb, ix, iy, Iv);
+            accumulate(0, ix, iy, Iv);
+        } else {
+            // ---- Scharr on the tap grid: 5 dp4a per pixel, zero outside the image ----
+#pragma unroll
+            for (int r = 0; r < C::DROUND; ++r) {
+                const int t = r * 32 + lane;
+                if (t < C::DTASK) {
+                    const int gy = t / C::DSEG, gx0 = (t - gy * C::DSEG) * 8;
+                    const int off = gy * C::PS + mis + gx0;      // byte of pixel (gx0-1, gy-1)
+                    const int sh8 = (off & 3) * 8;
+                    int ix[8], iy[8];
+#pragma unroll
+                    for (int k = 0; k < 8; ++k) { ix[k] = 0; iy[k] = 0; }
+#pragma unroll
+                    for (int rr = 0; rr < 3; ++rr) {
+                        const uint32_t* w = reinterpret_cast<const uint32_t*>(patch + (off & ~3) + rr * C::PS);
+                        const uint32_t w0 = w[0], w1 = w[1], w2 = w[2], w3 = w[3];
+                        const uint32_t a0 = __funnelshift_r(w0, w1, sh8), a1 = __funnelshift_r(w1, w2, sh8), a2 = __funnelshift_r(w2, w3, sh8);
+                        uint32_t q[8];
+                        q[0] = a0; q[1] = __funnelshift_r(a0, a1, 8); q[2] = __funnelshift_r(a0, a1, 16); q[3] = __funnelshift_r(a0, a1, 24);
+                        q[4] = a1; q[5] = __funnelshift_r(a1, a2, 8); q[6] = __funnelshift_r(a1, a2, 16); q[7] = __funnelshift_r(a1, a2, 24);
+                        // q[k] = pixels (x-1, x, x+1, x+2) of row gy-1+rr for x = gx0+k
+                        const int cx = rr == 1 ? 0x000A00F6 : 0x000300FD;                  // (-10,0,10,0) / (-3,0,3,0)
+                        const int cy = rr == 0 ? 0x00FDF6FD : 0x00030A03;                  // (-3,-10,-3,0) / (3,10,3,0)
+#pragma unroll
+                        for (int k = 0; k < 8; ++k) {
+                            ix[k] = dp4a_us(q[k], cx, ix[k]);
+                            if (rr != 1) iy[k] = dp4a_us(q[k], cy, iy[k]);
+                        }
+                    }
+                    const int X0 = ipx + gx0, Y = ipy + gy;
+                    const bool rowok = Y >= 0 && Y < lh;
+                    if (!(rowok && X0 >= 0 && X0 + 7 < lw)) {
+#pragma unroll
+                        for (int k = 0; k < 8; ++k) {
+                            const bool ok = rowok && X0 + k >= 0 && X0 + k < lw;
+                            ix[k] = ok ? ix[k] : 0; iy[k] = ok ? iy[k] : 0;
+                        }
+                    }
+                    int4* dxp = reinterpret_cast<int4*>(derx + gy * C::DS + gx0);
+                    int4* dyp = reinterpret_cast<int4*>(dery + gy * C::DS + gx0);
+                    dxp[0] = make_int4(ix[0], ix[1], ix[2], ix[3]); dxp[1] = make_int4(ix[4], ix[5], ix[6], ix[7]);
+                    dyp[0] = make_int4(iy[0], iy[1], iy[2], iy[3]); dyp[1] = make_int4(iy[4], iy[5], iy[6], iy[7]);
+                }
+            }
+            __syncwarp();
+#pragma unroll
+            for (int r = 0; r < C::NROUND; ++r) {
+                const int off = (ty[r] + 1) * C::PS + mis + 1 + tx[r];
+                int Iv[8];
+                if (off & 4) interp_run8_64<C::PS, true>(patch_s, off, (off & 3) * 8, wt, wb, Iv);
+                else interp_run8_64<C::PS, false>(patch_s, off, (off & 3) * 8, wt, wb, Iv);
+                const int* d0 = derx + ty[r] * C::DS + tx[r];
+                const int* e0 = dery + ty[r] * C::DS + tx[r];
+                int dx0[9], dx1[9], dy0[9], dy1[9];
+                {
+                    const int4 p0 = *reinterpret_cast<const int4*>(d0), p1 = *reinterpret_cast<const int4*>(d0 + 4);
+                    const int4 q0 = *reinterpret_cast<const int4*>(d0 + C::DS), q1 = *reinterpret_cast<const int4*>(d0 + C::DS + 4);
+                    dx0[0] = p0.x; dx0[1] = p0.y; dx0[2] = p0.z; dx0[3] = p0.w; dx0[4] = p1.x; dx0[5] = p1.y; dx0[6] = p1.z; dx0[7] = p1.w; dx0[8] = d0[8];
+                    dx1[0] = q0.x; dx1[1] = q0.y; dx1[2] = q0.z; dx1[3] = q0.w; dx1[4] = q1.x; dx1[5] = q1.y; dx1[6] = q1.z; dx1[7] = q1.w; dx1[8] = d0[C::DS + 8];
+                    const int4 r0 = *reinterpret_cast<const int4*>(e0), r1 = *reinterpret_cast<const int4*>(e0 + 4);
+                    const int4 s0 = *reinterpret_cast<const int4*>(e0 + C::DS), s1 = *reinterpret_cast<const int4*>(e0 + C::DS + 4);
+                    dy0[0] = r0.x; dy0[1] = r0.y; dy0[2] = r0.z; dy0[3] = r0.w; dy0[4] = r1.x; dy0[5] = r1.y; dy0[6] = r1.z; dy0[7] = r1.w; dy0[8] = e0[8];
+                    dy1[0] = s0.x; dy1[1] = s0.y; dy1[2] = s0.z; dy1[3] = s0.w; dy1[4] = s1.x; dy1[5] = s1.y; dy1[6] = s1.z; dy1[7] = s1.w; dy1[8] = e0[C::DS + 8];
+                }
+                int ix[8], iy[8];
+#pragma unroll
+                for (int k = 0; k < 8; ++k) {
+                    ix[k] = (dx0[k] * iw00 + dx0[k + 1] * iw01 + dx1[k] * iw10 + dx1[k + 1] * iw11 + (1 << (W_BITS - 1))) >> W_BITS;
+                    iy[k] = (dy0[k] * iw00 + dy0[k + 1] * iw01 + dy1[k] * iw10 + dy1[k + 1] * iw11 + (1 << (W_BITS - 1))) >> W_BITS;
+                }
+                accumulate(r, ix, iy, Iv);
+            }
         }
+        const bool wide = __any_sync(0xffffffffu, max(sA11, sA22) > C::ITER_SUM_FAST_MAX);   // this level's iteration sums
         float A11, A12, A22, unused;
         warp_sum2_f32(sA11, sA22, A11, A22);
         warp_sum2_f32(sA12, 0, A12, unused);
@@ -454,7 +538,7 @@ klt_kernel_v3(const KltArgs a)
                 }
             }
             float b1, b2;
-            warp_sum2_f32(sb1, sb2, b1, b2);
+            warp_sum2_f32(sb1, sb2, wide, b1, b2);
             b1 = __fmul_rn(b1, FLT_SCALE); b2 = __fmul_rn(b2, FLT_SCALE);
             const float dx = __fmul_rn(__fsub_rn(__fmul_rn(A12, b2), __fmul_rn(A22, b1)), D);
             const float dy = __fmul_rn(__fsub_rn(__fmul_rn(A12, b1), __fmul_rn(A11, b2)), D);
@@ -481,6 +565,7 @@ klt_kernel_v3(const KltArgs a)
                 st = 0;
                 continue;
             }
+            if (!want_err) continue;
             bilinear_weights(__fsub_rn(qx, (float)inx), __fsub_rn(qy, (float)iny), iw00, iw01, iw10, iw11);
             unsigned ux = (unsigned)inx - (unsigned)xlo, uy = (unsigned)iny - (unsigned)ylo;
             if (ux > xspan || uy > yspan) {
