@@ -262,6 +262,17 @@ void b200vo_batch_destroy(b200vo_batch* b);
  * Synchronous (waits for the step in flight); touches nothing but the listed sequences' intrinsics.
  */
 int b200vo_batch_set_intrinsics(b200vo_batch* b, int n_seq, const int32_t* seqs, const double* K);
+/*
+ * Per-sequence frame size.  cfg->rows x cfg->cols is the size of a SLOT, the largest frame the batch accepts, and every
+ * frame array keeps the slot layout [batch][cfg->rows][cfg->cols].  b200vo_batch_create gives every sequence the slot size;
+ * this call gives each of the n_seq distinct sequences seqs[k] the frame size rows[k] x cols[k] (int32 [n_seq]): its image
+ * is the top-left rows[k] x cols[k] of its slot (row stride cfg->cols), the bytes to the right of and below it are never
+ * read, and it is tracked and detected exactly as in a batch of its own size (its own pyramid level count included).
+ * A size must fit the slot and be larger than the window (cfg->win_h x cfg->win_w).  Bad indices (out of range, repeated),
+ * n_seq < 1, null arrays, a bad size or submitted frame sets still waiting: B200VO_E_BADARG and nothing changes.
+ * The resident frames no longer match: the next step needs b200vo_batch_prime.  Synchronous.
+ */
+int b200vo_batch_set_frame_size(b200vo_batch* b, int n_seq, const int32_t* seqs, const int32_t* rows, const int32_t* cols);
 /* Upload the first frame of every sequence (frames: batch x rows x cols, tight). */
 int b200vo_batch_prime(b200vo_batch* b, const uint8_t* frames);
 /*
@@ -351,7 +362,12 @@ void b200vo_loop_destroy(b200vo_loop* lp);
  * before b200vo_loop_load or b200vo_loop_bootstrap of that slot.  Same validation (B200VO_E_BADARG, nothing changes).
  * Synchronous. */
 int b200vo_loop_set_intrinsics(b200vo_loop* lp, int n_seq, const int32_t* seqs, const double* K);
-/* State of sequence `seq` after its bootstrap (host arrays): frame uint8 (rows,cols) tight = the current frame;
+/* Per-sequence frame size of the loop, as b200vo_batch_set_frame_size (same validation: B200VO_E_BADARG, nothing changes).
+ * The listed sequences become B200VO_LOOP_IDLE: their state arrays stay readable, and steps skip them until
+ * b200vo_loop_load or b200vo_loop_bootstrap runs for them.  Synchronous. */
+int b200vo_loop_set_frame_size(b200vo_loop* lp, int n_seq, const int32_t* seqs, const int32_t* rows, const int32_t* cols);
+/* State of sequence `seq` after its bootstrap (host arrays): frame uint8 (rows,cols) tight at the sequence's own frame size
+ * (b200vo_loop_set_frame_size) = the current frame;
  * lm float32 (n_lm,3) + lm_kp float32 (n_lm,2); keys / first_keys float32 (n_cand,2) + first_pose int32 (n_cand)
  * = potential_keys / potential_first_keys / potential_transforms; poses double (n_poses,12) = self.transforms as
  * (R_CW row-major | t_CW).  The sequence's status becomes B200VO_LOOP_OK.  Synchronous. */
@@ -369,8 +385,9 @@ int b200vo_loop_load(b200vo_loop* lp, int seq, const uint8_t* frame, const float
  * state arrays, takes the status and is skipped by steps until it is loaded or bootstrapped again.  Sequences not listed
  * are untouched.  Bad indices (out of range, repeated), n_seq < 1 or null arrays: B200VO_E_BADARG before any device work.
  * A sequence whose RANSAC subset draw exhausts the fixed table of cv2 random numbers also gets NO_BOOTSTRAP.
- * Synchronous; synchronises the host twice per SIFT chunk of frames plus three times, and once more per workspace that
- * has to grow. */
+ * frames0 / frames1 keep the slot layout whatever the sequences' own frame sizes.
+ * Synchronous; synchronises the host twice per SIFT chunk of frames of each distinct frame size among the listed sequences
+ * plus three times, and once more per workspace that has to grow. */
 int b200vo_loop_bootstrap(b200vo_loop* lp, int n_seq, const int32_t* seqs, const uint8_t* frames0, const uint8_t* frames1,
                           double ratio, int32_t* status, int32_t* num_pts, int32_t* n_lm, int32_t* n_cand);
 /* The same arrays back (capacity-sized outputs: max_landmarks, max_candidates, max_frames rows), plus the counts and

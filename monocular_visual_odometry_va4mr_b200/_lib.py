@@ -104,6 +104,7 @@ SIGNATURES = {
     "b200vo_batch_create": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(BatchCfg), C.POINTER(C.c_void_p)]),
     "b200vo_batch_destroy": (None, [C.c_void_p]),
     "b200vo_batch_set_intrinsics": (C.c_int, [C.c_void_p, C.c_int, c_i32p, c_f64p]),
+    "b200vo_batch_set_frame_size": (C.c_int, [C.c_void_p, C.c_int, c_i32p, c_i32p, c_i32p]),
     "b200vo_batch_prime": (C.c_int, [C.c_void_p, c_u8p]),
     "b200vo_batch_submit_frames": (C.c_int, [C.c_void_p, c_u8p]),
     "b200vo_batch_submit_frames_dev": (C.c_int, [C.c_void_p, C.c_void_p]),
@@ -117,6 +118,7 @@ SIGNATURES = {
     "b200vo_loop_create": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(LoopCfg), C.POINTER(C.c_void_p)]),
     "b200vo_loop_destroy": (None, [C.c_void_p]),
     "b200vo_loop_set_intrinsics": (C.c_int, [C.c_void_p, C.c_int, c_i32p, c_f64p]),
+    "b200vo_loop_set_frame_size": (C.c_int, [C.c_void_p, C.c_int, c_i32p, c_i32p, c_i32p]),
     "b200vo_loop_load": (C.c_int, [C.c_void_p, C.c_int, c_u8p, c_f32p, c_f32p, C.c_int, c_f32p, c_f32p, c_i32p, C.c_int, c_f64p,
                                    C.c_int]),
     "b200vo_loop_read_state": (C.c_int, [C.c_void_p, C.c_int, c_f32p, c_f32p, c_i32p, c_f32p, c_f32p, c_i32p, c_i32p, c_f64p, c_i32p,

@@ -51,6 +51,41 @@ def _set_intrinsics(ctx, fn, h, batch, seqs, K, what):
         raise _lib.B200VOError(f"{what} failed ({rc}): {ctx.last_error()}")
 
 
+def _set_frame_size(ctx, fn, h, seqs, sizes, what):
+    """Shared body of SequenceBatch / VOBatch.set_frame_size.  -> (seqs, sizes) as the call took them."""
+    seqs = np.ascontiguousarray(seqs, np.int32).reshape(-1)
+    sizes = np.asarray(sizes)
+    if sizes.shape != (len(seqs), 2) or not np.issubdtype(sizes.dtype, np.integer):
+        raise ValueError(f"sizes must be integer (len(seqs) = {len(seqs)}, 2) (rows, cols), got {sizes.dtype} {sizes.shape}")
+    rows = np.ascontiguousarray(sizes[:, 0], np.int32)
+    cols = np.ascontiguousarray(sizes[:, 1], np.int32)
+    rc = fn(h, len(seqs), _p(seqs, c_i32p), _p(rows, c_i32p), _p(cols, c_i32p))
+    if rc == -1:
+        raise ValueError(f"{what}: {ctx.last_error()}")
+    if rc != 0:
+        raise _lib.B200VOError(f"{what} failed ({rc}): {ctx.last_error()}")
+    return seqs, np.stack([rows, cols], 1)
+
+
+def _pack_frames(frames, sizes, rows, cols, out=None):
+    """A list of per-sequence 2-D uint8 images, each of its sequence's (rows_s, cols_s), packed into the slot layout
+    (len, rows, cols); the bytes outside each image are zero.  An array is returned as it is."""
+    if not isinstance(frames, (list, tuple)):
+        return frames
+    if len(frames) != len(sizes):
+        raise ValueError(f"{len(frames)} frames for {len(sizes)} sequences")
+    if out is None:
+        out = np.zeros((len(frames), rows, cols), np.uint8)
+    else:
+        out[...] = 0
+    for k, (f, (r, c)) in enumerate(zip(frames, sizes)):
+        f = np.asarray(f)
+        if f.dtype != np.uint8 or f.shape != (r, c):
+            raise ValueError(f"frame {k} must be ({r}, {c}) uint8, got {f.dtype} {f.shape}")
+        out[k, :r, :c] = f
+    return out
+
+
 class _PinnedBlock:
     """Owner of one b200vo_host_alloc block.  The numpy arrays carved from it keep it alive (it hangs off the
     ctypes buffer that is the arrays' base), so a result array that outlives its SequenceBatch -- e.g.
@@ -82,10 +117,12 @@ class _PinnedBlock:
 class SequenceBatch:
     def __init__(self, batch, rows, cols, K, win=(15, 15), max_level=5, criteria=(3, 50, 0.01),
                  min_eig_thr=1e-4, pnp_iters=500, pnp_reproj_err=8.0, pnp_conf=0.99,
-                 max_landmarks=1024, max_candidates=1024, ctx: _lib.Context | None = None):
+                 max_landmarks=1024, max_candidates=1024, frame_size=None, ctx: _lib.Context | None = None):
         self.ctx = ctx or _lib.default_context(0)
         self.batch, self.rows, self.cols = int(batch), int(rows), int(cols)
         self.L, self.Cn = int(max_landmarks), int(max_candidates)
+        self.frame_size = np.tile(np.int32([self.rows, self.cols]), (self.batch, 1))   # (batch, 2) rows, cols of every sequence
+        self._submitted = []   # page-locked slot-layout copies of submitted frame lists, alive until their step
         cfg = BatchCfg()
         cfg.rows, cfg.cols = self.rows, self.cols
         cfg.win_w, cfg.win_h, cfg.max_level = int(win[0]), int(win[1]), int(max_level)
@@ -105,6 +142,8 @@ class SequenceBatch:
         self.h = h
         if K_rows is not None:
             self.set_intrinsics(np.arange(self.batch), K_rows)
+        if frame_size is not None:
+            self.set_frame_size(np.arange(self.batch), frame_size)
         # host outputs (reused, page-locked so that step() reads them back without a staging copy)
         b, L, Cn = self.batch, self.L, self.Cn
         self.lm_next = self.pinned_empty((b, L, 2), np.float32)
@@ -145,6 +184,19 @@ class SequenceBatch:
         entries, last row (0, 0, 1).  Bad shapes, indices or matrices raise ValueError and change nothing.  Synchronous."""
         _set_intrinsics(self.ctx, self.ctx.lib.b200vo_batch_set_intrinsics, self.h, self.batch, seqs, K, "b200vo_batch_set_intrinsics")
 
+    def set_frame_size(self, seqs, sizes):
+        """Give the distinct sequences ``seqs`` the frame sizes ``sizes`` (len(seqs), 2) int (rows, cols).  ``rows`` x ``cols`` of the
+        constructor is the slot, the largest frame: a sequence's image is the top-left of its slot in every frame array, and it is
+        tracked and detected exactly as in a batch of its own size.  A size must fit the slot and exceed the window.  Bad shapes,
+        indices or sizes, or submitted frames still waiting, raise ValueError and change nothing.  The next step needs prime().
+        Synchronous."""
+        seqs, sizes = _set_frame_size(self.ctx, self.ctx.lib.b200vo_batch_set_frame_size, self.h, seqs, sizes, "b200vo_batch_set_frame_size")
+        self.frame_size[seqs] = sizes
+
+    def _frames(self, frames):
+        """frames of a step: the slot-layout array, or a list of per-sequence 2-D images packed into it"""
+        return _pack_frames(frames, self.frame_size, self.rows, self.cols)
+
     def pinned_empty(self, shape, dtype) -> np.ndarray:
         """numpy array in page-locked host memory (b200vo_host_alloc): DMA'd in place by step()."""
         dt = np.dtype(dtype)
@@ -160,13 +212,17 @@ class SequenceBatch:
         """(n_sets, batch, rows, cols) uint8 array in page-locked memory (b200vo_host_alloc)."""
         return self.pinned_empty((n_sets, self.batch, self.rows, self.cols), np.uint8)
 
-    def prime(self, frames: np.ndarray):
-        frames = np.ascontiguousarray(frames, np.uint8).reshape(self.batch, self.rows, self.cols)
+    def prime(self, frames):
+        frames = np.ascontiguousarray(self._frames(frames), np.uint8).reshape(self.batch, self.rows, self.cols)
         self._chk(self.ctx.lib.b200vo_batch_prime(self.h, _p(frames, c_u8p)), "b200vo_batch_prime")
 
-    def submit_frames(self, frames: np.ndarray):
-        """Hand over the frames of a FUTURE step (page-locked array from pinned_frames()): their upload and
-        pyramid build overlap the step in flight; the step called with frames=None consumes them."""
+    def submit_frames(self, frames):
+        """Hand over the frames of a FUTURE step (page-locked array from pinned_frames(), or a list of per-sequence images,
+        packed into a page-locked copy): their upload and pyramid build overlap the step in flight; the step called with
+        frames=None consumes them."""
+        if isinstance(frames, (list, tuple)):
+            frames = _pack_frames(frames, self.frame_size, self.rows, self.cols, self.pinned_frames()[0])
+            self._submitted = (self._submitted + [frames])[-3:]
         assert frames.dtype == np.uint8 and frames.flags.c_contiguous and frames.size == self.batch * self.rows * self.cols
         self._chk(self.ctx.lib.b200vo_batch_submit_frames(self.h, _p(frames, c_u8p)), "b200vo_batch_submit_frames")
 
@@ -180,6 +236,8 @@ class SequenceBatch:
         the next step() overwrites them (copy what must survive it); they remain valid memory after close().
         frames=None: use the oldest frame set given to submit_frames()."""
         b, L, Cn = self.batch, self.L, self.Cn
+        if frames is not None:
+            frames = self._frames(frames)
         assert frames is None or (frames.dtype == np.uint8 and frames.flags.c_contiguous and frames.size == b * self.rows * self.cols)
         assert lm_pts.dtype == np.float32 and lm_pts.shape == (b, L, 2) and lm_pts.flags.c_contiguous
         assert lm_obj.dtype == np.float32 and lm_obj.shape == (b, L, 3) and lm_obj.flags.c_contiguous
@@ -260,9 +318,11 @@ class VOBatch:
     OK, IDLE, FEW_POINTS, PNP_FAILED, OVERFLOW, DETECT_LIMIT, NO_BOOTSTRAP = range(7)
 
     def __init__(self, batch, rows, cols, K, options, max_landmarks=4096, max_candidates=8192, max_frames=1024,
-                 ctx: _lib.Context | None = None):
+                 frame_size=None, ctx: _lib.Context | None = None):
         self.ctx = ctx or _lib.default_context(0)
         self.batch, self.rows, self.cols = int(batch), int(rows), int(cols)
+        self.frame_size = np.tile(np.int32([self.rows, self.cols]), (self.batch, 1))   # (batch, 2) rows, cols of every sequence
+        self._submitted = []
         self.L, self.Cn, self.P = int(max_landmarks), int(max_candidates), int(max_frames)
         self.options = options
         K, K_rows = _batch_K(K, self.batch)
@@ -274,6 +334,8 @@ class VOBatch:
         self.h = h
         if K_rows is not None:
             self.set_intrinsics(np.arange(self.batch), K_rows)
+        if frame_size is not None:
+            self.set_frame_size(np.arange(self.batch), frame_size)
         b = self.batch
         self._res = dict(status=self.pinned_empty((b,), np.int32), n_inliers=self.pinned_empty((b,), np.int32),
                          n_lm=self.pinned_empty((b,), np.int32), n_cand=self.pinned_empty((b,), np.int32),
@@ -316,13 +378,26 @@ class VOBatch:
         pass ``K`` to them).  Bad shapes, indices or matrices raise ValueError and change nothing.  Synchronous."""
         _set_intrinsics(self.ctx, self.ctx.lib.b200vo_loop_set_intrinsics, self.h, self.batch, seqs, K, "b200vo_loop_set_intrinsics")
 
+    def set_frame_size(self, seqs, sizes):
+        """Give the distinct sequences ``seqs`` the frame sizes ``sizes`` (len(seqs), 2) int (rows, cols).  ``rows`` x ``cols`` of the
+        constructor is the slot, the largest frame: a sequence's image is the top-left of its slot in the frames of ``step``,
+        ``submit_frames`` and ``bootstrap`` (which also take a list of per-sequence images), and each sequence runs exactly as in
+        a batch of its own size.  The listed sequences become IDLE (state kept, skipped by ``step``) until ``load`` or
+        ``bootstrap``.  A size must fit the slot and exceed the window.  Bad shapes, indices or sizes, or submitted frames
+        still waiting, raise ValueError and change nothing.  Synchronous."""
+        seqs, sizes = _set_frame_size(self.ctx, self.ctx.lib.b200vo_loop_set_frame_size, self.h, seqs, sizes, "b200vo_loop_set_frame_size")
+        self.frame_size[seqs] = sizes
+
     def load(self, seq: int, frame: np.ndarray, state: dict, K=None):
         """Set sequence ``seq`` to ``state`` (see the class docstring) with ``frame`` as its current frame; its status
         becomes OK.  ``K`` (3, 3): the sequence's camera from now on (``set_intrinsics`` first).  Out-of-range counts or
         first_pose values raise ValueError and change nothing."""
         f = np.ascontiguousarray(frame, np.uint8)
-        if f.shape != (self.rows, self.cols):
-            raise ValueError(f"frame must be ({self.rows}, {self.cols}) uint8")
+        if not 0 <= int(seq) < self.batch:
+            raise ValueError(f"seq = {seq} is outside [0, batch = {self.batch})")
+        r, c = (int(v) for v in self.frame_size[int(seq)])
+        if f.shape != (r, c):
+            raise ValueError(f"frame must be ({r}, {c}) uint8: the sequence's frame size")
         lm = np.ascontiguousarray(state['lm'], np.float32).reshape(-1, 3)
         kp = np.ascontiguousarray(state['lm_kp'], np.float32).reshape(-1, 2)
         keys = np.ascontiguousarray(state['keys'], np.float32).reshape(-1, 2)
@@ -351,6 +426,11 @@ class VOBatch:
         bootstrapped again.  ``K`` (len(seqs), 3, 3): the listed sequences' cameras from now on (``set_intrinsics`` first).
         Bad indices, frame shapes or K raise ValueError and change nothing.  Synchronous."""
         seqs = np.arange(self.batch, dtype=np.int32) if seqs is None else np.ascontiguousarray(seqs, np.int32).reshape(-1)
+        if isinstance(frames0, (list, tuple)) or isinstance(frames1, (list, tuple)):
+            if ((seqs < 0) | (seqs >= self.batch)).any():
+                raise ValueError(f"seqs must lie in [0, batch = {self.batch})")
+            frames0 = _pack_frames(list(frames0), self.frame_size[seqs], self.rows, self.cols)
+            frames1 = _pack_frames(list(frames1), self.frame_size[seqs], self.rows, self.cols)
         f0 = np.ascontiguousarray(frames0, np.uint8)
         f1 = np.ascontiguousarray(frames1, np.uint8)
         shape = (len(seqs), self.rows, self.cols)
@@ -381,8 +461,12 @@ class VOBatch:
         return dict(lm=lm[:nl], lm_kp=kp[:nl], keys=keys[:nc], first_keys=fk[:nc], first_pose=fp[:nc], poses=poses[:npo],
                     status=status.value)
 
-    def submit_frames(self, frames: np.ndarray):
-        """Frames of a FUTURE step (page-locked, from pinned_frames()); step(None) consumes them, oldest first."""
+    def submit_frames(self, frames):
+        """Frames of a FUTURE step (page-locked, from pinned_frames(), or a list of per-sequence images, packed into a page-locked
+        copy); step(None) consumes them, oldest first."""
+        if isinstance(frames, (list, tuple)):
+            frames = _pack_frames(frames, self.frame_size, self.rows, self.cols, self.pinned_frames()[0])
+            self._submitted = (self._submitted + [frames])[-3:]
         assert frames.dtype == np.uint8 and frames.flags.c_contiguous and frames.size == self.batch * self.rows * self.cols
         self._chk(self.ctx.lib.b200vo_loop_submit_frames(self.h, _p(frames, c_u8p)), "b200vo_loop_submit_frames")
 
@@ -391,11 +475,12 @@ class VOBatch:
         self._chk(self.ctx.lib.b200vo_loop_submit_frames_dev(self.h, frames_dev), "b200vo_loop_submit_frames_dev")
 
     def step(self, frames=None) -> dict:
-        """One frame for every sequence (frames (batch, rows, cols) uint8; None: the oldest submitted set).  Synchronous.
+        """One frame for every sequence (frames (batch, rows, cols) uint8 in the slot layout, or a list of per-sequence images;
+        None: the oldest submitted set).  Synchronous.
         Returns views on REUSED page-locked arrays: status, n_inliers, n_lm, n_cand int32 (batch,) and pose_cw float64
         (batch, 12), the pose appended this step (0 unless status is OK)."""
         if frames is not None:
-            frames = np.ascontiguousarray(frames, np.uint8)
+            frames = np.ascontiguousarray(_pack_frames(frames, self.frame_size, self.rows, self.cols), np.uint8)
             assert frames.size == self.batch * self.rows * self.cols
         self._chk(self.ctx.lib.b200vo_loop_step(self.h, _p(frames, c_u8p) if frames is not None else None, *self._res_ptrs),
                   "b200vo_loop_step")

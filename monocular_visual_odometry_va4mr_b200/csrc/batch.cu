@@ -123,6 +123,12 @@ extern "C" int b200vo_batch_create(b200vo_ctx* ctx, int batch, const b200vo_batc
     }
     if (rc) { b200vo_batch_destroy(B); return rc; }
     B->intr = (const VoIntrinsics*)B->intr_buf.p;
+    // every sequence starts with the slot size (no table on the device until a sequence is given another)
+    B->ext_host.resize(batch);
+    vo_seq_ext(cfg->rows, cfg->cols, cfg->win_w, cfg->win_h, cfg->max_level, &B->ext_host[0]);
+    for (int k = 1; k < batch; ++k) B->ext_host[k] = B->ext_host[0];
+    rc = vo_reserve(ctx, B->ext_buf, (size_t)batch * sizeof(VoSeqExt));
+    if (rc) { b200vo_batch_destroy(B); return rc; }
     *out = B;
     return 0;
 }
@@ -143,6 +149,48 @@ int batch_set_intrinsics(b200vo_batch* B, int n_seq, const int32_t* seqs, const 
 extern "C" int b200vo_batch_set_intrinsics(b200vo_batch* B, int n_seq, const int32_t* seqs, const double* K)
 {
     return B ? batch_set_intrinsics(B, n_seq, seqs, K) : B200VO_E_BADARG;
+}
+
+int batch_set_frame_size(b200vo_batch* B, int n_seq, const int32_t* seqs, const int32_t* rows, const int32_t* cols)
+{
+    b200vo_ctx* ctx = B->ctx;
+    const b200vo_batch_cfg& c = B->cfg;
+    if (n_seq < 1 || n_seq > B->batch) return vo_set_err(ctx, B200VO_E_BADARG, "n_seq = %d is outside [1, batch = %d]", n_seq, B->batch);
+    if (!seqs || !rows || !cols) return vo_set_err(ctx, B200VO_E_BADARG, "null array");
+    std::vector<char> seen(B->batch, 0);
+    for (int k = 0; k < n_seq; ++k) {
+        if (seqs[k] < 0 || seqs[k] >= B->batch)
+            return vo_set_err(ctx, B200VO_E_BADARG, "seqs[%d] = %d is outside [0, batch = %d)", k, seqs[k], B->batch);
+        if (seen[seqs[k]]++) return vo_set_err(ctx, B200VO_E_BADARG, "sequence %d is listed twice", seqs[k]);
+        // the slot bounds the frame; the window bounds it from below as it bounds cfg->rows / cfg->cols (and with it the
+        // detector's 3 x 3 minimum)
+        if (rows[k] > c.rows || cols[k] > c.cols)
+            return vo_set_err(ctx, B200VO_E_BADARG, "sequence %d: %d x %d does not fit the %d x %d slot", seqs[k], rows[k], cols[k], c.rows, c.cols);
+        if (rows[k] <= c.win_h || cols[k] <= c.win_w)
+            return vo_set_err(ctx, B200VO_E_BADARG, "sequence %d: %d x %d is not larger than the %d x %d window", seqs[k], rows[k], cols[k],
+                              c.win_h, c.win_w);
+    }
+    if (B->q_count > 0) return vo_set_err(ctx, B200VO_E_BADARG, "submitted frame sets are waiting: their pyramids were built at the old sizes");
+    std::vector<VoSeqExt> ext = B->ext_host;
+    for (int k = 0; k < n_seq; ++k) vo_seq_ext(rows[k], cols[k], c.win_w, c.win_h, c.max_level, &ext[seqs[k]]);
+    bool uniform = true;
+    for (const VoSeqExt& e : ext) uniform = uniform && e.w[0] == c.cols && e.h[0] == c.rows;
+    VO_CUDA(ctx, cudaSetDevice(ctx->device));
+    VO_CUDA(ctx, cudaStreamSynchronize(ctx->stream));   // no step in flight reads the rows
+    VO_CUDA(ctx, cudaStreamSynchronize(B->pre_stream));
+    VO_CUDA(ctx, cudaMemcpyAsync(B->ext_buf.p, ext.data(), ext.size() * sizeof(VoSeqExt), cudaMemcpyHostToDevice, ctx->stream));
+    VO_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    B->ext_host.swap(ext);
+    B->ext = uniform ? nullptr : (const VoSeqExt*)B->ext_buf.p;
+    return 0;
+}
+
+extern "C" int b200vo_batch_set_frame_size(b200vo_batch* B, int n_seq, const int32_t* seqs, const int32_t* rows, const int32_t* cols)
+{
+    if (!B) return B200VO_E_BADARG;
+    VO_TRY(batch_set_frame_size(B, n_seq, seqs, rows, cols));
+    B->primed = false;   // the resident pyramids were built at the old sizes
+    return 0;
 }
 
 __global__ void trace_stamp_kernel(unsigned long long* dst)
@@ -207,7 +255,7 @@ extern "C" void b200vo_batch_destroy(b200vo_batch* B)
     kill_stream(B->io_stream);
     kill_stream(B->pose_stream);
     for (auto& s : B->slabs) if (s.p) cudaFree(s.p);
-    for (DevBuf* d : {&B->raw, &B->raw_pre, &B->pts_in, &B->outs, &B->work, &B->gftt_ws, &B->intr_buf}) if (d->p) cudaFree(d->p);
+    for (DevBuf* d : {&B->raw, &B->raw_pre, &B->pts_in, &B->outs, &B->work, &B->gftt_ws, &B->intr_buf, &B->ext_buf}) if (d->p) cudaFree(d->p);
     for (auto& e : B->q_ev) kill_event(e);
     for (auto& e : B->chunk_ev) kill_event(e);
     for (auto& e : B->copy_ev) kill_event(e);
@@ -234,7 +282,7 @@ static int batch_upload_frames(b200vo_batch* B, const uint8_t* frames, int slab_
     }
     VO_CUDA(ctx, cudaMemcpyAsync(B->raw.p, src, total, cudaMemcpyHostToDevice, ctx->stream));
     VO_TRY(vo_build_pyramids(ctx, (const uint8_t*)B->raw.p, fb, B->cfg.rows, B->cfg.cols, B->geom,
-                             (uint8_t*)B->slabs[slab_set].p, B->geom.slab_bytes, B->batch, ctx->stream));
+                             (uint8_t*)B->slabs[slab_set].p, B->geom.slab_bytes, B->batch, ctx->stream, batch_ext_dev(B, 0), batch_ext_host(B, 0)));
     return 0;
 }
 
@@ -307,7 +355,8 @@ int batch_issue_prefetch(b200vo_batch* B, cudaEvent_t after, bool wait_step_end)
             raw = (const uint8_t*)B->raw_pre.p;
         }
         VO_TRY(vo_build_pyramids(ctx, raw, fb, B->cfg.rows, B->cfg.cols, B->geom,
-                                 (uint8_t*)B->slabs[B->q_set[slot]].p, B->geom.slab_bytes, B->batch, B->pre_stream));
+                                 (uint8_t*)B->slabs[B->q_set[slot]].p, B->geom.slab_bytes, B->batch, B->pre_stream, batch_ext_dev(B, 0),
+                                 batch_ext_host(B, 0)));
         VO_CUDA(ctx, cudaEventRecord(B->q_ev[slot], B->pre_stream));
         B->q_src[slot] = nullptr;
     }
@@ -347,7 +396,7 @@ static int batch_track(b200vo_batch* B, cudaStream_t stream, int b0, int nb, con
         if (whole) prof_mark(B, 0, stream);
         if (frames_dev)
             VO_TRY(vo_build_pyramids(ctx, frames_dev + (size_t)b0 * fb, fb, c.rows, c.cols, B->geom,
-                                     (uint8_t*)B->slabs[nxt].p + (size_t)b0 * sb, sb, nb, stream));
+                                     (uint8_t*)B->slabs[nxt].p + (size_t)b0 * sb, sb, nb, stream, batch_ext_dev(B, b0), batch_ext_host(B, b0)));
         if (whole) { prof_mark(B, 1, stream); B->prof_row_open = B->profile && B->prof_n < B200VO_PROF_RING; }
     }
     KltPointSet sets[2] = {{L, n_lm + b0, lm_pts + (size_t)b0 * L * 2, lm_next + (size_t)b0 * L * 2, lm_status + (size_t)b0 * L, nullptr},
@@ -357,7 +406,7 @@ static int batch_track(b200vo_batch* B, cudaStream_t stream, int b0, int nb, con
     const KltPointSet* first = which == 2 ? sets + 1 : sets;
     const int n_sets = which == 0 ? (Cn > 0 ? 2 : 1) : 1;   // which 1, 4: landmark set; 2: candidate set
     VO_TRY(vo_klt_launch2(ctx, B->geom, (const uint8_t*)B->slabs[B->cur].p + (size_t)b0 * sb, sb,
-                          (const uint8_t*)B->slabs[nxt].p + (size_t)b0 * sb, sb, nb, first, n_sets, 0, B->kp, stream));
+                          (const uint8_t*)B->slabs[nxt].p + (size_t)b0 * sb, sb, nb, first, n_sets, 0, B->kp, stream, batch_ext_dev(B, b0)));
     return 0;
 }
 
@@ -776,7 +825,7 @@ extern "C" int b200vo_batch_good_features(b200vo_batch* B, int max_corners, doub
     float* d_out = nullptr;
     int* d_small = nullptr;
     VO_TRY(vo_gftt_batch_launch(ctx, (const uint8_t*)B->slabs[B->cur].p + B->geom.off[0], B->geom.slab_bytes, B->geom.pitch[0], c.rows, c.cols,
-                                nb, max_corners, quality, min_dist, B->gftt_ws.p, &d_out, &d_small));
+                                nb, max_corners, quality, min_dist, B->gftt_ws.p, &d_out, &d_small, B->ext));
     const size_t b_out = vo_align((size_t)max_corners * 8, 256);
     const size_t out_bytes = b_out * nb, small_bytes = (size_t)nb * VO_GFTT_SMALL * sizeof(int);
     VO_TRY(vo_reserve_pinned(ctx, out_bytes + small_bytes));

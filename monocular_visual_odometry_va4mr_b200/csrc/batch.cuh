@@ -47,6 +47,12 @@ struct b200vo_batch {
     DevBuf intr_buf;
     const VoIntrinsics* intr = nullptr;
     std::vector<VoIntrinsics> intr_host;
+    // the frame size of every sequence (b200vo_batch_set_frame_size): device rows read by the pyramid, tracker and detector
+    // kernels, host mirror of them.  `ext` is nullptr while every sequence has the slot size cfg.rows x cfg.cols: the
+    // kernels then take the slot geometry from their launch arguments, as a batch without per-sequence sizes always did.
+    DevBuf ext_buf;
+    const VoSeqExt* ext = nullptr;
+    std::vector<VoSeqExt> ext_host;
     // host-input path: frames arrive chunk by chunk on a copy stream while earlier chunks are tracked
     cudaStream_t chunk_stream[B200VO_BATCH_STREAMS] = {};  // chunk k: H2D -> pyramid -> KLT on stream k % STREAMS
     cudaEvent_t chunk_ev[B200VO_BATCH_CHUNKS] = {};
@@ -80,3 +86,9 @@ int batch_track_pose_overlapped(b200vo_batch* B, const uint8_t* frames_dev, cons
 int batch_finish(b200vo_batch* B);
 // Validates the (index, K) pairs and, only when all are valid, waits for the work in flight and uploads the new rows (synchronous)
 int batch_set_intrinsics(b200vo_batch* B, int n_seq, const int32_t* seqs, const double* K);
+// Validates the (index, rows, cols) triples and, only when all are valid and no submitted frame set waits, waits for the
+// work in flight and uploads the new extents (synchronous)
+int batch_set_frame_size(b200vo_batch* B, int n_seq, const int32_t* seqs, const int32_t* rows, const int32_t* cols);
+// the device rows of sequences [b0, ...) and their host copy, or nullptr for both while every sequence has the slot size
+inline const VoSeqExt* batch_ext_dev(const b200vo_batch* B, int b0) { return B->ext ? B->ext + b0 : nullptr; }
+inline const VoSeqExt* batch_ext_host(const b200vo_batch* B, int b0) { return B->ext ? B->ext_host.data() + b0 : nullptr; }

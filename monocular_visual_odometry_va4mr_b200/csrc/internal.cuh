@@ -30,6 +30,15 @@ struct PyrGeom {
     size_t slab_bytes;
 };
 
+// The extents of one sequence's frames inside a batch whose slot (PyrGeom) may be larger: its level count and the
+// size of every level by the (w + 1) / 2 chain.  Its image is the top-left w[0] x h[0] of the slot, with the slot's
+// row pitch; nothing to the right of or below a level's REFLECT_101 ring is ever read.  A device array of [batch] rows
+// per batch object whose sequences do not all have the slot size; kernels given none use the slot's own geometry.
+struct VoSeqExt {
+    int levels;
+    int w[VO_MAX_LEVELS], h[VO_MAX_LEVELS];
+};
+
 struct KltParams {
     int win_w, win_h;
     int max_count;
@@ -154,16 +163,23 @@ __device__ __forceinline__ int cta_compact(int n, Keep keep, Emit emit)
 int vo_pyr_levels(int w, int h, int win_w, int win_h, int max_level);
 void vo_pyr_geom(int rows, int cols, int levels, PyrGeom* g);
 Pyramid vo_pyramid_at(const PyrGeom& g, uint8_t* slab);
-// raw (tight, device) -> bordered level 0, then levels 1..L-1; `batch` slabs/raws strided.
+// the extents of a rows x cols frame with the level count cv2 builds for it
+void vo_seq_ext(int rows, int cols, int win_w, int win_h, int max_level, VoSeqExt* e);
+// raw (device, rows of `raw_row` bytes, 0: cols) -> bordered level 0, then levels 1..L-1; `batch` slabs/raws strided.
+// d_ext / h_ext: [batch] per-sequence extents on the device and their host copy (both or neither), each inside the
+// slot geometry g; every level of a sequence is built at its own size, levels beyond its own count are not built.
 int vo_build_pyramids(b200vo_ctx* ctx, const uint8_t* d_raw, size_t raw_stride, int rows, int cols,
-                      const PyrGeom& g, uint8_t* d_slab, size_t slab_stride, int batch, cudaStream_t stream);
+                      const PyrGeom& g, uint8_t* d_slab, size_t slab_stride, int batch, cudaStream_t stream,
+                      const VoSeqExt* d_ext = nullptr, const VoSeqExt* h_ext = nullptr, size_t raw_row = 0);
 
 // ---- gftt.cu: detection on device-resident bordered level-0 images, one per batch entry ----
 #define VO_GFTT_SMALL 4          // ints per image in the result block: max bits | n candidates | n corners | spare
 #define VO_GFTT_BATCH_CAP 32768  // candidates per image the batched path can rank
 size_t vo_gftt_batch_workspace(int rows, int cols, int batch, int max_corners);
+// d_ext: [batch] per-sequence extents (level 0 is read), nullptr: every image is rows x cols
 int vo_gftt_batch_launch(b200vo_ctx* ctx, const uint8_t* d_img0, size_t img_stride, int pitch, int rows, int cols, int batch,
-                         int max_corners, double quality, double min_dist, void* ws, float** d_corners_out, int** d_small_out);
+                         int max_corners, double quality, double min_dist, void* ws, float** d_corners_out, int** d_small_out,
+                         const VoSeqExt* d_ext = nullptr);
 
 // ---- klt.cu ----
 struct KltPointSet {
@@ -175,10 +191,11 @@ struct KltPointSet {
     float* err;         // [batch][cap] or nullptr
 };
 void vo_klt_trace_read(b200vo_ctx* ctx, std::vector<unsigned long long>& out);   // B200VO_TRACE_FILE aid
-// Tracks the points of up to two sets in `batch` independent frame pairs, on `stream`.
+// Tracks the points of up to two sets in `batch` independent frame pairs, on `stream`.  d_ext: [batch] per-sequence
+// extents (nullptr: every sequence has the geometry g)
 int vo_klt_launch2(b200vo_ctx* ctx, const PyrGeom& g, const uint8_t* d_prev_slab, size_t prev_stride,
                    const uint8_t* d_next_slab, size_t next_stride, int batch, const KltPointSet* sets, int n_sets,
-                   int n_fixed, const KltParams& kp, cudaStream_t stream);
+                   int n_fixed, const KltParams& kp, cudaStream_t stream, const VoSeqExt* d_ext = nullptr);
 
 // ---- knn.cu: device-resident kNN(k=2) + ratio test on the ctx stream (descriptors float32 [n][128])
 size_t vo_knn2_workspace(const b200vo_ctx* ctx, int nq, int nt);   // the scratch vo_knn2_ratio_dev reserves

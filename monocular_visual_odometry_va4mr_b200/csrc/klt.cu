@@ -23,6 +23,7 @@ struct KltArgs {
     unsigned long long off[VO_MAX_LEVELS];
     int w[VO_MAX_LEVELS], h[VO_MAX_LEVELS], pitch[VO_MAX_LEVELS];
     int levels;
+    const VoSeqExt* ext;    // [batch] per-sequence level counts and level sizes, nullptr: levels / w / h above for every sequence
     int batch, n_fixed;
     // up to two point sets per sequence (landmark keypoints, candidate keypoints): [batch][cap[s]]
     int cap[2];
@@ -66,7 +67,8 @@ __device__ __forceinline__ void bilinear_weights(float a, float b, int& w00, int
     w11 = (1 << W_BITS) - w00 - w01 - w10;
 }
 
-template <int WW, int WH>
+// EXT: the sequences have their own level counts and level sizes (a.ext); otherwise a.levels / a.w / a.h hold for all
+template <int WW, int WH, bool EXT>
 __global__ void __launch_bounds__(KLT_WARPS * 32)
 klt_kernel(const KltArgs a)
 {
@@ -103,15 +105,17 @@ klt_kernel(const KltArgs a)
     float outx = 0.f, outy = 0.f;
     int st = 1;
     float e = 0.f;
+    const int levels = EXT ? a.ext[seq].levels : a.levels;
 
-    for (int level = a.levels - 1; level >= 0; --level) {
-        const int lw = a.w[level], lh = a.h[level], pitch = a.pitch[level];
+    for (int level = levels - 1; level >= 0; --level) {
+        const int lw = EXT ? a.ext[seq].w[level] : a.w[level], lh = EXT ? a.ext[seq].h[level] : a.h[level];
+        const int pitch = a.pitch[level];
         const uint8_t* I = prev + a.off[level];
         const uint8_t* J = next + a.off[level];
         const float sc = (float)(1.0 / (double)(1 << level));
         float ppx = __fmul_rn(px0, sc), ppy = __fmul_rn(py0, sc);
         float nx, ny;
-        if (level == a.levels - 1) { nx = ppx; ny = ppy; }
+        if (level == levels - 1) { nx = ppx; ny = ppy; }
         else { nx = __fmul_rn(outx, 2.f); ny = __fmul_rn(outy, 2.f); }
         outx = nx; outy = ny;
         ppx = __fsub_rn(ppx, hwx); ppy = __fsub_rn(ppy, hwy);
@@ -264,7 +268,7 @@ klt_kernel(const KltArgs a)
 
 int vo_klt_launch2(b200vo_ctx* ctx, const PyrGeom& g, const uint8_t* d_prev_slab, size_t prev_stride,
                    const uint8_t* d_next_slab, size_t next_stride, int batch, const KltPointSet* sets, int n_sets,
-                   int n_fixed, const KltParams& kp, cudaStream_t stream)
+                   int n_fixed, const KltParams& kp, cudaStream_t stream, const VoSeqExt* d_ext)
 {
     if (batch <= 0 || n_sets <= 0) return 0;
     KltArgs a{};
@@ -274,6 +278,7 @@ int vo_klt_launch2(b200vo_ctx* ctx, const PyrGeom& g, const uint8_t* d_prev_slab
     for (int l = 0; l < g.levels; ++l) {
         a.off[l] = g.off[l]; a.w[l] = g.w[l]; a.h[l] = g.h[l]; a.pitch[l] = g.pitch[l];
     }
+    a.ext = d_ext;
     a.batch = batch; a.n_fixed = n_fixed;
     for (int s = 0; s < 2; ++s) {
         const bool on = s < n_sets;
@@ -297,15 +302,23 @@ int vo_klt_launch2(b200vo_ctx* ctx, const PyrGeom& g, const uint8_t* d_prev_slab
     size_t smem = (size_t)a.smem_per_warp * KLT_WARPS;
     const long long total_warps = (long long)batch * (a.cap[0] + a.cap[1]);
     const unsigned grid = (unsigned)((total_warps + KLT_WARPS - 1) / KLT_WARPS);
-    void (*kern)(const KltArgs) = klt_kernel<0, 0>;
+    void (*kern)(const KltArgs) = d_ext ? klt_kernel<0, 0, true> : klt_kernel<0, 0, false>;
+    bool staged = false;
     // the staged kernel (persistent warps + work queue) for the two window sizes it is built for; the queue counter is
     // an int, so a launch of 2^30 features or more takes the generic kernel (same arithmetic, same results)
     const bool sized = (kp.win_w == 21 && kp.win_h == 21) || (kp.win_w == 15 && kp.win_h == 15);
     unsigned launch_grid = grid;
     if (sized && total_warps < (1ll << 30)) {
         int min_ctas;
-        if (kp.win_w == 21) { kern = klt_kernel_v3<21, 21>; smem = (size_t)KV3<21, 21>::PER_WARP * KLT_WARPS + 64; min_ctas = KV3<21, 21>::MIN_CTAS; }
-        else { kern = klt_kernel_v3<15, 15>; smem = (size_t)KV3<15, 15>::PER_WARP * KLT_WARPS + 64; min_ctas = KV3<15, 15>::MIN_CTAS; }
+        staged = true;
+        // per-sequence extents: the instances that read them (a uniform batch keeps the ones that take the launch's geometry)
+        if (kp.win_w == 21) {
+            kern = d_ext ? klt_kernel_v3<21, 21, true> : klt_kernel_v3<21, 21, false>;
+            smem = (size_t)KV3<21, 21>::PER_WARP * KLT_WARPS + 64; min_ctas = KV3<21, 21>::MIN_CTAS;
+        } else {
+            kern = d_ext ? klt_kernel_v3<15, 15, true> : klt_kernel_v3<15, 15, false>;
+            smem = (size_t)KV3<15, 15>::PER_WARP * KLT_WARPS + 64; min_ctas = KV3<15, 15>::MIN_CTAS;
+        }
         if (!ctx->d_klt_queue.p) {
             VO_TRY(vo_reserve(ctx, ctx->d_klt_queue, (size_t)KLT_QUEUE_SLOTS * KLT_QUEUE_INTS * sizeof(int)));
             VO_CUDA(ctx, cudaMemsetAsync(ctx->d_klt_queue.p, 0, (size_t)KLT_QUEUE_SLOTS * KLT_QUEUE_INTS * sizeof(int), stream));
@@ -325,9 +338,9 @@ int vo_klt_launch2(b200vo_ctx* ctx, const PyrGeom& g, const uint8_t* d_prev_slab
         if (!seen) {
             if (smem > 48 * 1024)
                 VO_CUDA(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            if (kern != klt_kernel<0, 0>)   // the staged kernels live in shared memory: let 8 CTAs (64 registers each) fit
+            if (staged)   // the staged kernels live in shared memory: let 8 CTAs (64 registers each) fit
                 VO_CUDA(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-            if (free_slot >= 0 && kern != klt_kernel<0, 0>) configured[free_slot] = (void*)kern;   // the generic kernel's smem size varies per call
+            if (free_slot >= 0 && staged) configured[free_slot] = (void*)kern;   // the generic kernel's smem size varies per call
         }
     }
     kern<<<launch_grid, KLT_WARPS * 32, smem, stream>>>(a);

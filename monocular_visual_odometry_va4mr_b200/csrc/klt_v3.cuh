@@ -223,7 +223,8 @@ __device__ __forceinline__ void template_interior(uint32_t patch_s, int row_off,
     }
 }
 
-template <int WW, int WH>
+// EXT: the sequences have their own level counts and level sizes (a.ext); otherwise a.levels / a.w / a.h hold for all
+template <int WW, int WH, bool EXT>
 __global__ void __launch_bounds__(KLT_WARPS * 32, (KV3<WW, WH>::MIN_CTAS))
 klt_kernel_v3(const KltArgs a)
 {
@@ -299,18 +300,20 @@ klt_kernel_v3(const KltArgs a)
     int pb = 0, pf_level = -1;     // patch buffer in use; level whose patch was prefetched into it
     cp_async_wait_pending(0);      // nothing of the previous feature may still be landing in this warp's buffers
     __syncwarp();
+    const VoSeqExt* ext = EXT ? a.ext + seq : nullptr;
+    const int levels = EXT ? ext->levels : a.levels;
 
-    for (int level = a.levels - 1; level >= 0; --level) {
+    for (int level = levels - 1; level >= 0; --level) {
         int lw, lh;
-        asm volatile("mov.s32 %0, %1;" : "=r"(lw) : "r"(a.w[level]));
-        asm volatile("mov.s32 %0, %1;" : "=r"(lh) : "r"(a.h[level]));
+        asm volatile("mov.s32 %0, %1;" : "=r"(lw) : "r"(EXT ? ext->w[level] : a.w[level]));
+        asm volatile("mov.s32 %0, %1;" : "=r"(lh) : "r"(EXT ? ext->h[level] : a.h[level]));
         const int pitch = a.pitch[level];
         const uint8_t* I = prev + a.off[level];
         const uint8_t* J = next + a.off[level];
         const float sc = __int_as_float((127 - level) << 23);   // exactly 2^-level
         float ppx = __fmul_rn(px0, sc), ppy = __fmul_rn(py0, sc);
         float nx, ny;
-        if (level == a.levels - 1) { nx = ppx; ny = ppy; }
+        if (level == levels - 1) { nx = ppx; ny = ppy; }
         else { nx = __fmul_rn(outx, 2.f); ny = __fmul_rn(outy, 2.f); }
         outx = nx; outy = ny;
         ppx = __fsub_rn(ppx, hwx); ppy = __fsub_rn(ppy, hwy);
@@ -361,7 +364,7 @@ klt_kernel_v3(const KltArgs a)
             const int nl = level - 1;
             const float sc2 = __int_as_float((127 - nl) << 23);
             const int qx = floor_to_int(__fsub_rn(__fmul_rn(px0, sc2), hwx)), qy = floor_to_int(__fsub_rn(__fmul_rn(py0, sc2), hwy));
-            if (!(qx < -WW || qx >= a.w[nl] || qy < -WH || qy >= a.h[nl])) {
+            if (!(qx < -WW || qx >= (EXT ? ext->w[nl] : a.w[nl]) || qy < -WH || qy >= (EXT ? ext->h[nl] : a.h[nl]))) {
                 const uint8_t* n0 = prev + a.off[nl] + (long long)(qy - 1) * a.pitch[nl] + (qx - 1);
                 const int m3 = (int)(reinterpret_cast<uintptr_t>(n0) & 7);
                 stage_rows_async8<C::PSLOT, C::PROWS>(wbase_s + (pb ^ 1) * C::B_PATCH, n0 - m3, a.pitch[nl], lane);

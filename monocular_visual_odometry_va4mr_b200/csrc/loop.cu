@@ -286,7 +286,7 @@ static int loop_core(b200vo_loop* lp, const uint8_t* frames_dev, const LoopOut& 
     int* small = nullptr;
     VO_TRY(vo_gftt_batch_launch(ctx, (const uint8_t*)B->slabs[B->nxt].p + B->geom.off[0], B->geom.slab_bytes, B->geom.pitch[0],
                                 c.batch.rows, c.batch.cols, nb, c.max_corners, c.quality_level, c.feature_min_dist, B->gftt_ws.p,
-                                &corners, &small));
+                                &corners, &small, B->ext));
     d.corners = corners; d.gftt_small = small;
     loop_commit_kernel<<<nb, LOOP_T, 0, ctx->stream>>>(d, o);
     ctx->launches++;
@@ -382,11 +382,14 @@ extern "C" int b200vo_loop_load(b200vo_loop* lp, int seq, const uint8_t* frame, 
     VO_CUDA(ctx, cudaSetDevice(ctx->device));
     VO_CUDA(ctx, cudaStreamSynchronize(ctx->stream));   // no step in flight reads the state
     cudaStream_t st = ctx->stream;
-    const size_t fb = (size_t)lp->cfg.batch.rows * lp->cfg.batch.cols, sb = B->geom.slab_bytes;
+    const int rows = lp->cfg.batch.rows, cols = lp->cfg.batch.cols;
+    const size_t fb = (size_t)rows * cols, sb = B->geom.slab_bytes;
+    // the frame is tight at the sequence's own size: it becomes the top-left of a slot-layout frame
+    const int rs = B->ext_host[seq].h[0], cs = B->ext_host[seq].w[0];
     VO_TRY(vo_reserve(ctx, B->raw, fb));
-    VO_CUDA(ctx, cudaMemcpyAsync(B->raw.p, frame, fb, cudaMemcpyHostToDevice, st));
-    VO_TRY(vo_build_pyramids(ctx, (const uint8_t*)B->raw.p, fb, lp->cfg.batch.rows, lp->cfg.batch.cols, B->geom,
-                             (uint8_t*)B->slabs[B->cur].p + (size_t)seq * sb, sb, 1, st));
+    VO_CUDA(ctx, cudaMemcpy2DAsync(B->raw.p, (size_t)cols, frame, (size_t)cs, (size_t)cs, (size_t)rs, cudaMemcpyHostToDevice, st));
+    VO_TRY(vo_build_pyramids(ctx, (const uint8_t*)B->raw.p, fb, rows, cols, B->geom,
+                             (uint8_t*)B->slabs[B->cur].p + (size_t)seq * sb, sb, 1, st, batch_ext_dev(B, seq), batch_ext_host(B, seq)));
     const size_t lo = (size_t)seq * d.L, co = (size_t)seq * d.C;
     if (n_lm > 0) {
         VO_CUDA(ctx, cudaMemcpyAsync(d.lm + 3 * lo, lm, (size_t)n_lm * 12, cudaMemcpyHostToDevice, st));
@@ -408,6 +411,23 @@ extern "C" int b200vo_loop_load(b200vo_loop* lp, int seq, const uint8_t* frame, 
 extern "C" int b200vo_loop_set_intrinsics(b200vo_loop* lp, int n_seq, const int32_t* seqs, const double* K)
 {
     return lp ? batch_set_intrinsics(lp->B, n_seq, seqs, K) : B200VO_E_BADARG;
+}
+
+extern "C" int b200vo_loop_set_frame_size(b200vo_loop* lp, int n_seq, const int32_t* seqs, const int32_t* rows, const int32_t* cols)
+{
+    if (!lp) return B200VO_E_BADARG;
+    b200vo_ctx* ctx = lp->ctx;
+    VO_TRY(batch_set_frame_size(lp->B, n_seq, seqs, rows, cols));
+    // the listed sequences' pyramids no longer match their frames: IDLE (state arrays kept) until loaded or bootstrapped
+    const int idle = B200VO_LOOP_IDLE, zero = 0;
+    const LoopDev& d = lp->d;
+    for (int k = 0; k < n_seq; ++k) {
+        VO_CUDA(ctx, cudaMemcpyAsync(d.status + seqs[k], &idle, 4, cudaMemcpyHostToDevice, ctx->stream));
+        VO_CUDA(ctx, cudaMemcpyAsync(d.trk_lm + seqs[k], &zero, 4, cudaMemcpyHostToDevice, ctx->stream));
+        VO_CUDA(ctx, cudaMemcpyAsync(d.trk_cand + seqs[k], &zero, 4, cudaMemcpyHostToDevice, ctx->stream));
+    }
+    VO_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    return 0;
 }
 
 extern "C" int b200vo_loop_read_state(b200vo_loop* lp, int seq, float* lm, float* lm_kp, int32_t* n_lm, float* keys, float* first_keys,
@@ -569,19 +589,53 @@ extern "C" int b200vo_loop_bootstrap(b200vo_loop* lp, int n_seq, const int32_t* 
     }
     const int rows = lp->cfg.batch.rows, cols = lp->cfg.batch.cols;
     const size_t fb = (size_t)rows * cols, sb = B->geom.slab_bytes, ns = n_seq;
+    // The sequences run in groups of one frame size (SIFT works on one size per call), the groups in the order of their
+    // first listed sequence, the sequences of a group in list order: position j of the run is listed sequence perm[j].
+    // Every per-sequence result depends on the sequence alone, so the order changes nothing but where it is stored.
+    std::vector<int> perm, grp_end;
+    {
+        std::vector<char> done(ns, 0);
+        for (int k = 0; k < n_seq; ++k) {
+            if (done[k]) continue;
+            const VoSeqExt& e = B->ext_host[seqs[k]];
+            for (int i = k; i < n_seq; ++i) {
+                const VoSeqExt& f = B->ext_host[seqs[i]];
+                if (!done[i] && f.w[0] == e.w[0] && f.h[0] == e.h[0]) { done[i] = 1; perm.push_back(i); }
+            }
+            grp_end.push_back((int)perm.size());
+        }
+    }
+    bool in_order = true;
+    for (int j = 0; j < n_seq; ++j) in_order = in_order && perm[j] == j;
+    std::vector<int32_t> seq_run(ns);
+    for (int j = 0; j < n_seq; ++j) seq_run[j] = seqs[perm[j]];
+    seqs = seq_run.data();
     VO_CUDA(ctx, cudaSetDevice(ctx->device));
     VO_CUDA(ctx, cudaStreamSynchronize(ctx->stream));   // no step in flight reads the state
     cudaStream_t st = ctx->stream;
-    // the two frames of sequence k are frames 2k and 2k + 1 of the SIFT batch
+    // the two frames of sequence j of the run are frames 2j and 2j + 1 of the SIFT batch (slot layout)
     const size_t b_raw = vo_align(ns * 2 * fb, 256), b_cnt = vo_align(ns * 8, 256);
     VO_TRY(vo_reserve(ctx, lp->boot_in, b_raw + 2 * b_cnt));
     uint8_t* raw = (uint8_t*)lp->boot_in.p;
     int* d_nkp = (int*)(raw + b_raw);
     int* d_row = (int*)(raw + b_raw + b_cnt);
-    VO_CUDA(ctx, cudaMemcpy2DAsync(raw, 2 * fb, frames0, fb, fb, ns, cudaMemcpyHostToDevice, st));
-    VO_CUDA(ctx, cudaMemcpy2DAsync(raw + fb, 2 * fb, frames1, fb, fb, ns, cudaMemcpyHostToDevice, st));
+    if (in_order) {
+        VO_CUDA(ctx, cudaMemcpy2DAsync(raw, 2 * fb, frames0, fb, fb, ns, cudaMemcpyHostToDevice, st));
+        VO_CUDA(ctx, cudaMemcpy2DAsync(raw + fb, 2 * fb, frames1, fb, fb, ns, cudaMemcpyHostToDevice, st));
+    } else {
+        for (int j = 0; j < n_seq; ++j) {
+            VO_CUDA(ctx, cudaMemcpyAsync(raw + 2 * j * fb, frames0 + (size_t)perm[j] * fb, fb, cudaMemcpyHostToDevice, st));
+            VO_CUDA(ctx, cudaMemcpyAsync(raw + (2 * j + 1) * fb, frames1 + (size_t)perm[j] * fb, fb, cudaMemcpyHostToDevice, st));
+        }
+    }
+    // SIFT per size group, each group's keypoint and descriptor rows after the previous group's
     int n_rows = 0;
-    VO_TRY(vo_sift_frames(ctx, raw, fb, 2 * n_seq, rows, cols, true, d_nkp, d_row, &n_rows));
+    for (size_t g = 0, j0 = 0; g < grp_end.size(); j0 = grp_end[g++]) {
+        const VoSeqExt& e = B->ext_host[seqs[j0]];
+        const int m = grp_end[g] - (int)j0;
+        VO_TRY(vo_sift_frames(ctx, raw + 2 * j0 * fb, fb, 2 * m, e.h[0], e.w[0], true, d_nkp + 2 * j0, d_row + 2 * j0, &n_rows, n_rows,
+                              (size_t)cols));
+    }
     std::vector<int> h_cnt(4 * ns);
     VO_CUDA(ctx, cudaMemcpyAsync(h_cnt.data(), d_nkp, ns * 8, cudaMemcpyDeviceToHost, st));
     VO_CUDA(ctx, cudaMemcpyAsync(h_cnt.data() + 2 * ns, d_row, ns * 8, cudaMemcpyDeviceToHost, st));
@@ -601,7 +655,7 @@ extern "C" int b200vo_loop_bootstrap(b200vo_loop* lp, int n_seq, const int32_t* 
     const size_t nc = ns * cap, sq = std::max(sum_q, 1);
     const size_t sizes[] = {ns * BT_KINDS * 4, sq * 8, sq * 8, sq, nc * 8, nc * 8, ns * 4, ns * 72, nc, ns * 16, ns * 4,
                             nc * 8, nc * 8, ns * 4, nc * 4, ns * 384, ns * 16, ns * 96, ns * 8, ns * 96, ns * 4, ns * 4, ns * 96,
-                            nc, nc * 12, nc * 12, nc * 8, ns * 4, ns * 4, ns * 16, ns * sb, ns * sizeof(VoIntrinsics)};
+                            nc, nc * 12, nc * 12, nc * 8, ns * 4, ns * 4, ns * 16, ns * sb, ns * sizeof(VoSeqExt), ns * sizeof(VoIntrinsics)};
     size_t total = 0;
     for (size_t x : sizes) total += vo_align(x, 256);
     VO_TRY(vo_reserve(ctx, lp->boot_ws, total));
@@ -631,6 +685,7 @@ extern "C" int b200vo_loop_bootstrap(b200vo_loop* lp, int n_seq, const int32_t* 
     t.n_new = (int*)take(); t.flags = (int*)take();
     b.res = (int*)take();
     uint8_t* slab = (uint8_t*)take();
+    VoSeqExt* ext_run = (VoSeqExt*)take();
     // the camera of each listed sequence, in list order (the bootstrap's kernels take the sequence from the grid)
     VoIntrinsics* intr = (VoIntrinsics*)take();
     std::vector<VoIntrinsics> h_intr(ns);
@@ -677,16 +732,21 @@ extern "C" int b200vo_loop_bootstrap(b200vo_loop* lp, int n_seq, const int32_t* 
     t.n = b.tri_n; t.n_poses = one; t.cur = b.cur;
     t.first_keys = b.inl0; t.keys = b.inl1; t.first_pose = zeros; t.poses = first_pose_cw;
     VO_TRY(vo_triangulate_batch_launch(ctx, t, n_seq, st));
-    VO_TRY(vo_build_pyramids(ctx, raw + fb, 2 * fb, rows, cols, B->geom, slab, sb, n_seq, st));
+    // the second frames' pyramids, each at its sequence's size (the run's own table; none while every size is the slot's)
+    std::vector<VoSeqExt> h_ext(ns);
+    for (int j = 0; j < n_seq; ++j) h_ext[j] = B->ext_host[seqs[j]];
+    if (B->ext) VO_CUDA(ctx, cudaMemcpyAsync(ext_run, h_ext.data(), ns * sizeof(VoSeqExt), cudaMemcpyHostToDevice, st));
+    VO_TRY(vo_build_pyramids(ctx, raw + fb, 2 * fb, rows, cols, B->geom, slab, sb, n_seq, st, B->ext ? ext_run : nullptr,
+                             B->ext ? h_ext.data() : nullptr));
     boot_load_kernel<<<n_seq, LOOP_T, 0, st>>>(lp->d, b);
     ctx->launches++;
     VO_CUDA(ctx, cudaGetLastError());
     std::vector<int> h_res(4 * ns);
     VO_CUDA(ctx, cudaMemcpyAsync(h_res.data(), b.res, ns * 16, cudaMemcpyDeviceToHost, st));
     VO_CUDA(ctx, cudaStreamSynchronize(st));
-    memcpy(status, h_res.data(), ns * 4);
-    memcpy(num_pts, h_res.data() + ns, ns * 4);
-    memcpy(n_lm, h_res.data() + 2 * ns, ns * 4);
-    memcpy(n_cand, h_res.data() + 3 * ns, ns * 4);
+    for (int j = 0; j < n_seq; ++j) {   // back to list order
+        const int k = perm[j];
+        status[k] = h_res[j]; num_pts[k] = h_res[ns + j]; n_lm[k] = h_res[2 * ns + j]; n_cand[k] = h_res[3 * ns + j];
+    }
     return 0;
 }

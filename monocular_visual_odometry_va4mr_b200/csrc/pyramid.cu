@@ -39,6 +39,16 @@ void vo_pyr_geom(int rows, int cols, int levels, PyrGeom* g)
     g->slab_bytes = vo_align(off, 256) + 256;
 }
 
+void vo_seq_ext(int rows, int cols, int win_w, int win_h, int max_level, VoSeqExt* e)
+{
+    *e = VoSeqExt{};
+    e->levels = vo_pyr_levels(cols, rows, win_w, win_h, max_level);
+    for (int l = 0; l < e->levels; ++l) {
+        e->w[l] = cols; e->h[l] = rows;
+        cols = (cols + 1) / 2; rows = (rows + 1) / 2;
+    }
+}
+
 Pyramid vo_pyramid_at(const PyrGeom& g, uint8_t* slab)
 {
     Pyramid p;
@@ -59,19 +69,21 @@ __device__ __forceinline__ int reflect101(int p, int len)
     return p;
 }
 
-// raw tight image -> bordered level 0.  One thread = one 16-byte store of the bordered row.
+// raw image (rows of raw_row bytes) -> bordered level 0.  One thread = one 16-byte store of the bordered row.
+// ext: the sequence's own width and height (the grid covers the slot's)
 __global__ void __launch_bounds__(256)
-pad_level0_kernel(const uint8_t* __restrict__ raw, size_t raw_stride, int w, int h,
-                  uint8_t* __restrict__ slab, size_t slab_stride, size_t off0, int pitch)
+pad_level0_kernel(const uint8_t* __restrict__ raw, size_t raw_stride, size_t raw_row, int w, int h,
+                  uint8_t* __restrict__ slab, size_t slab_stride, size_t off0, int pitch, const VoSeqExt* __restrict__ ext)
 {
     const int seq = blockIdx.z;
+    if (ext) { w = ext[seq].w[0]; h = ext[seq].h[0]; }
     const uint8_t* src = raw + seq * raw_stride;
     uint8_t* dst = slab + seq * slab_stride + off0;
     const int gx = (blockIdx.x * blockDim.x + threadIdx.x) * 16 - VO_BORDER;  // first of 16 px
     const int gy = blockIdx.y * blockDim.y + threadIdx.y - VO_BORDER;
     if (gx >= w + VO_BORDER || gy >= h + VO_BORDER) return;
     const int sy = reflect101(gy, h);
-    const uint8_t* srow = src + (size_t)sy * w;
+    const uint8_t* srow = src + (size_t)sy * raw_row;
     uint32_t v[4];
     if (gx >= 0 && gx + 15 < w) {
 #pragma unroll
@@ -101,9 +113,14 @@ pad_level0_kernel(const uint8_t* __restrict__ raw, size_t raw_stride, int w, int
 // bordered destination row; 5x5 binomial [1 4 6 4 1]^2, (sum+128)>>8.
 __global__ void __launch_bounds__(256)
 pyr_down_kernel(const uint8_t* __restrict__ slab_src, uint8_t* __restrict__ slab_dst, size_t slab_stride,
-                size_t off_s, int sw, int sh, int spitch, size_t off_d, int dw, int dh, int dpitch)
+                size_t off_s, int sw, int sh, int spitch, size_t off_d, int dw, int dh, int dpitch,
+                const VoSeqExt* __restrict__ ext, int level)
 {
     const int seq = blockIdx.z;
+    if (ext) {   // the sequence's own level `level` from its level - 1; nothing beyond its level count
+        if (level >= ext[seq].levels) return;
+        dw = ext[seq].w[level]; dh = ext[seq].h[level];
+    }
     const uint8_t* src = slab_src + seq * slab_stride + off_s;
     uint8_t* dst = slab_dst + seq * slab_stride + off_d;
     const int gx = (blockIdx.x * blockDim.x + threadIdx.x) * 4 - VO_BORDER;
@@ -161,13 +178,19 @@ pyr_down_kernel(const uint8_t* __restrict__ slab_src, uint8_t* __restrict__ slab
 
 __global__ void __launch_bounds__(256)
 pyr_down_tma_kernel(const __grid_constant__ CUtensorMap src_map, uint8_t* __restrict__ slab_dst, size_t slab_stride,
-                    size_t off_d, int dw, int dh, int dpitch, int fuse_border)
+                    size_t off_d, int dw, int dh, int dpitch, int fuse_border, const VoSeqExt* __restrict__ ext, int level)
 {
     // source bytes [0,160) and [128,288) of each row; each half starts on a 128-byte boundary (TMA destination)
     __shared__ __align__(128) uint8_t tile[2][(PD_SR * PD_SB + 127) / 128 * 128];
     __shared__ __align__(8) unsigned long long bar;
     const int seq = blockIdx.z;
     const int X0 = blockIdx.x * PD_TW, Y0 = blockIdx.y * PD_TH;
+    if (ext) {   // the sequence's own extents of this level: tiles outside them (and levels beyond its count) exit
+        if (level >= ext[seq].levels) return;
+        dw = ext[seq].w[level]; dh = ext[seq].h[level];
+        if (X0 >= dw || Y0 >= dh) return;
+        fuse_border = dw >= VO_BORDER + 2 && dh >= VO_BORDER + 2;
+    }
     const uint32_t bar_a = smem_u32(&bar);
     if (threadIdx.x == 0) {
         mbar_init(bar_a, 1);
@@ -240,9 +263,16 @@ pyr_down_tma_kernel(const __grid_constant__ CUtensorMap src_map, uint8_t* __rest
 // tracker's window reads depend on it)
 struct BorderArgs { int levels; int w[VO_MAX_LEVELS], h[VO_MAX_LEVELS], pitch[VO_MAX_LEVELS]; unsigned long long off[VO_MAX_LEVELS]; };
 __global__ void __launch_bounds__(256)
-pyr_border_level_kernel(uint8_t* __restrict__ slab, size_t slab_stride, BorderArgs a, int level)
+pyr_border_level_kernel(uint8_t* __restrict__ slab, size_t slab_stride, BorderArgs a, int level, const VoSeqExt* __restrict__ ext)
 {
-    const int w = a.w[level], h = a.h[level], pitch = a.pitch[level];
+    int w = a.w[level], h = a.h[level];
+    const int pitch = a.pitch[level];
+    if (ext) {   // only the sequences whose level was not given its ring by the tiles
+        const VoSeqExt& e = ext[blockIdx.z];
+        if (level >= e.levels) return;
+        w = e.w[level]; h = e.h[level];
+        if (w >= VO_BORDER + 2 && h >= VO_BORDER + 2) return;
+    }
     uint8_t* base = slab + blockIdx.z * slab_stride + a.off[level];
     // ring in aligned 4-byte words: top + bottom bands over the full bordered width, then per interior
     // row 8 words on the left (x = -32..-1) and 9 on the right (from x = w & ~3, covering w .. w+31)
@@ -292,14 +322,16 @@ static int pyr_src_map(b200vo_ctx* ctx, CUtensorMap* map, uint8_t* d_slab, size_
 }
 
 int vo_build_pyramids(b200vo_ctx* ctx, const uint8_t* d_raw, size_t raw_stride, int rows, int cols,
-                      const PyrGeom& g, uint8_t* d_slab, size_t slab_stride, int batch, cudaStream_t stream)
+                      const PyrGeom& g, uint8_t* d_slab, size_t slab_stride, int batch, cudaStream_t stream,
+                      const VoSeqExt* d_ext, const VoSeqExt* h_ext, size_t raw_row)
 {
+    if (!raw_row) raw_row = (size_t)cols;
     {
         dim3 block(32, 8);
         int gxn = (cols + 2 * VO_BORDER + 15) / 16;
         dim3 grid((gxn + block.x - 1) / block.x, (rows + 2 * VO_BORDER + block.y - 1) / block.y, batch);
-        pad_level0_kernel<<<grid, block, 0, stream>>>(d_raw, raw_stride, cols, rows, d_slab, slab_stride,
-                                                       g.off[0], g.pitch[0]);
+        pad_level0_kernel<<<grid, block, 0, stream>>>(d_raw, raw_stride, raw_row, cols, rows, d_slab, slab_stride,
+                                                       g.off[0], g.pitch[0], d_ext);
         ctx->launches++;
     }
     if (g.levels > 1) {
@@ -312,14 +344,20 @@ int vo_build_pyramids(b200vo_ctx* ctx, const uint8_t* d_raw, size_t raw_stride, 
                 VO_TRY(pyr_src_map(ctx, &map, d_slab, batch == 1 ? g.slab_bytes : slab_stride, batch, g, l - 1));
                 dim3 grid((g.w[l] + PD_TW - 1) / PD_TW, (g.h[l] + PD_TH - 1) / PD_TH, batch);
                 fused = g.w[l] >= VO_BORDER + 2 && g.h[l] >= VO_BORDER + 2;   // single-bounce reflection: the tiles write the ring
-                pyr_down_tma_kernel<<<grid, 256, 0, stream>>>(map, d_slab, slab_stride, g.off[l], g.w[l], g.h[l], g.pitch[l], fused ? 1 : 0);
+                pyr_down_tma_kernel<<<grid, 256, 0, stream>>>(map, d_slab, slab_stride, g.off[l], g.w[l], g.h[l], g.pitch[l], fused ? 1 : 0,
+                                                              d_ext, l);
+                if (h_ext) {   // the single-bounce test per sequence: a ring is left to the border kernel if any tile set could not write it
+                    fused = true;
+                    for (int b = 0; b < batch; ++b)
+                        if (l < h_ext[b].levels && !(h_ext[b].w[l] >= VO_BORDER + 2 && h_ext[b].h[l] >= VO_BORDER + 2)) fused = false;
+                }
             } else {
                 dim3 block(32, 8);
                 int gxn = (g.w[l] + 2 * VO_BORDER + 3) / 4;
                 dim3 grid((gxn + block.x - 1) / block.x, (g.h[l] + 2 * VO_BORDER + block.y - 1) / block.y, batch);
                 pyr_down_kernel<<<grid, block, 0, stream>>>(d_slab, d_slab, slab_stride, g.off[l - 1], g.w[l - 1],
                                                              g.h[l - 1], g.pitch[l - 1], g.off[l], g.w[l], g.h[l],
-                                                             g.pitch[l]);
+                                                             g.pitch[l], d_ext, l);
             }
             ctx->launches++;
             if (tma_ok && !fused) {
@@ -329,7 +367,7 @@ int vo_build_pyramids(b200vo_ctx* ctx, const uint8_t* d_raw, size_t raw_stride, 
                 for (int k = 0; k <= l; ++k) { ba.w[k] = g.w[k]; ba.h[k] = g.h[k]; ba.pitch[k] = g.pitch[k]; ba.off[k] = g.off[k]; }
                 // only level l needs filling now: launch with a single y-slice mapped onto level l
                 ba.levels = l + 1;
-                pyr_border_level_kernel<<<dim3(16, 1, batch), 256, 0, stream>>>(d_slab, slab_stride, ba, l);
+                pyr_border_level_kernel<<<dim3(16, 1, batch), 256, 0, stream>>>(d_slab, slab_stride, ba, l, d_ext);
                 ctx->launches++;
             }
         }

@@ -649,9 +649,10 @@ static int sift_reserve_keep(b200vo_ctx* ctx, DevBuf& b, size_t used, size_t byt
 }
 
 int vo_sift_frames(b200vo_ctx* ctx, const uint8_t* d_raw, size_t raw_stride, int n_frames, int rows, int cols, bool want_desc,
-                   int* d_n_frame, int* d_first_row, int* n_rows)
+                   int* d_n_frame, int* d_first_row, int* n_rows, int row0, size_t row_stride)
 {
     const int L = SIFT_LAYERS;
+    if (!row_stride) row_stride = (size_t)cols;
     SiftGeom G;
     sift_geom(rows, cols, G);
     const size_t per_frame = sift_per_frame_bytes(G);
@@ -666,7 +667,7 @@ int vo_sift_frames(b200vo_ctx* ctx, const uint8_t* d_raw, size_t raw_stride, int
     const float sg = 1.6f;
     const float sig_diff = sqrtf(std::max(sg * sg - 0.5f * 0.5f * 4, 0.01f));     // createInitialImage: float arithmetic
     const size_t fs = G.frame_bytes / 4;   // frame stride of the workspace, in floats
-    int base = 0;                          // output rows written so far
+    int base = row0;                       // output rows written so far
     for (int f0 = 0; f0 < n_frames; f0 += chunk) {
         const int nf = std::min(chunk, n_frames - f0);
         const size_t cand_cap = (size_t)nf * SIFT_CAND_CAP, kp_cap = (size_t)nf * SIFT_KP_CAP;
@@ -679,7 +680,7 @@ int vo_sift_frames(b200vo_ctx* ctx, const uint8_t* d_raw, size_t raw_stride, int
         float* up = (float*)(ws + G.o_up);
         float* tmp = (float*)(ws + G.o_tmp);
         sift_upscale_kernel<<<dim3((G.bcols + 255) / 256, G.brows, nf), 256, 0, ctx->stream>>>(d_raw + (size_t)f0 * raw_stride, rows, cols,
-                                                                                              (size_t)cols, raw_stride, up, fs);
+                                                                                              row_stride, raw_stride, up, fs);
         ctx->launches++;
         SiftPyrDev P{};
         P.fstride = fs;
