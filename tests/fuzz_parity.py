@@ -1,7 +1,7 @@
 """Randomised differential run: CUDA path (through the C ABI) vs the oracle, many shapes / sizes / seeds.
 Not collected by pytest (it runs for minutes); prints every mismatch.
 
-  python tests/fuzz_parity.py [seconds]          (FUZZ_SEED=n for another stream)
+  python tests/fuzz_parity.py [seconds]          (FUZZ_SEED=n for another stream, FUZZ_KINDS=batch for the batch kind alone)
 
 Round-1 record: 240 s on a B200 = 632 tracker calls (random image sizes 120..900 x 90..500, six window
 sizes, maxLevel 0..6, all three criteria types, points on quarter-pixel grids and with 3.2e-5 offsets),
@@ -12,7 +12,12 @@ Seed 4 (330 s, 3 372 calls) and seed 6 on the final round-1 binary (300 s, 3 012
 Round 2 (SIFT added; persistent tracker, fused pose kernel, second kNN kernel): seed 11 (180 s) one findEssentialMat case with
 4 mask points -- an ill-conditioned sample on which cv2 sides with the CUDA path (DESIGN.md section 2 fact 5; the oracle's
 root termination was aligned afterwards); seeds 21 and 22 (240 s each, 1 700 + 1 800 calls incl. 303 SIFT frames of random
-sizes) and, after the last kernel changes (branch-free kNN scan, tracker queue fix), seeds 31 and 32 (3 450 calls): 0 mismatches."""
+sizes) and, after the last kernel changes (branch-free kNN scan, tracker queue fix), seeds 31 and 32 (3 450 calls): 0 mismatches.
+Round 3 (the batch kind: SequenceBatch with per-sequence frame sizes, compared per sequence with the oracle on its own image;
+random slots up to 519 x 1299, 1-8 sequences of random and near-minimal sizes, the six windows, maxLevel 0..7, all three criteria
+types, zero or random padding, two tracker steps and one detection): FUZZ_KINDS=batch, seeds 41 and 42, 250 s each, run side by
+side on one B200 = 496 + 467 batches, 7 600 + 7 352 per-sequence tracker comparisons, 2 222 + 2 153 per-sequence detections:
+0 mismatches."""
 import os
 import sys
 import time
@@ -23,15 +28,108 @@ import numpy as np  # noqa: E402
 
 import oracle  # noqa: E402
 from make_golden import make_emat_pair, make_pnp_case, sift_like  # noqa: E402
-from monocular_visual_odometry_va4mr_b200 import cv2_compat, hotpath, synth  # noqa: E402
+from monocular_visual_odometry_va4mr_b200 import _lib, cv2_compat, hotpath, synth  # noqa: E402
+from monocular_visual_odometry_va4mr_b200.batch import SequenceBatch  # noqa: E402
+
+WINDOWS = [(15, 15), (21, 21), (9, 13), (31, 31), (5, 7), (21, 15)]
+
+
+def batch_case(rng, bad, stats):
+    """SequenceBatch with per-sequence frame sizes: a random slot, random sizes (near-minimal ones included), window,
+    maxLevel, criteria and padding; two tracker steps and one detection, each sequence against the oracle on its own image."""
+    win = WINDOWS[int(rng.integers(0, len(WINDOWS)))]
+    slot = (int(rng.integers(win[1] + 1, 520)), int(rng.integers(win[0] + 1, 1300)))
+    ml = int(rng.integers(0, 8))
+    crit = (int(rng.choice([1, 2, 3])), int(rng.integers(1, 40)), float(rng.choice([0.01, 0.03, 0.001])))
+    b = int(rng.integers(1, 9))
+
+    def dim(lo, hi):          # near-minimal, near-full or anywhere
+        u = rng.random()
+        return int(rng.integers(lo, min(lo + 4, hi) + 1)) if u < 0.3 else hi - int(rng.integers(0, 3)) if u < 0.45 else int(rng.integers(lo, hi + 1))
+    sizes = [(dim(win[1] + 1, slot[0]), dim(win[0] + 1, slot[1])) for _ in range(b)]
+    sizes = [(max(win[1] + 1, r), max(win[0] + 1, c)) for r, c in sizes]
+    full = synth.render_sequence(str(rng.choice(["kitti", "parking", "malaga"])), 3, seed=int(rng.integers(0, 1000)),
+                                 width=slot[1], height=slot[0], start=int(rng.integers(0, 5)))["frames"]
+    crops = []
+    for r, c in sizes:
+        y0, x0 = int(rng.integers(0, slot[0] - r + 1)), int(rng.integers(0, slot[1] - c + 1))
+        crops.append(np.ascontiguousarray(full[:, y0:y0 + r, x0:x0 + c]))
+    random_pad = rng.random() < 0.5
+
+    def layout(f):
+        out = rng.integers(0, 256, (b,) + slot, dtype=np.uint8) if random_pad else np.zeros((b,) + slot, np.uint8)
+        for k, im in enumerate(crops):
+            out[k, :im.shape[1], :im.shape[2]] = im[f]
+        return out
+
+    pts = []
+    for r, c in sizes:
+        n = int(rng.integers(1, 600))
+        p = np.column_stack([rng.uniform(-20, c + 20, n), rng.uniform(-20, r + 20, n)]).astype(np.float32)
+        if rng.random() < 0.5:
+            p = np.rint(p * 4) / 4
+        if rng.random() < 0.3:
+            p += np.float32(3.2e-5)
+        pts.append(np.ascontiguousarray(p, np.float32))
+    L = max(len(p) for p in pts)
+    lm = np.zeros((b, L, 2), np.float32)
+    for k, p in enumerate(pts):
+        lm[k, :len(p)] = p
+    cand = np.zeros_like(lm)
+    for k, p in enumerate(pts):
+        cand[k, :len(p)] = p[::-1]
+    n_pts = np.int32([len(p) for p in pts])
+    n_cand = np.int32([len(p) if rng.random() < 0.7 else 0 for p in pts])
+    cand_of = [np.ascontiguousarray(cand[k, :n_cand[k]]) for k in range(b)]
+    sb = SequenceBatch(b, *slot, synth.K_KITTI, win=win, max_level=ml, criteria=crit, max_landmarks=max(L, 4), max_candidates=L,
+                       frame_size=sizes)
+    obj = np.zeros((b, max(L, 4), 3), np.float32)
+    lm4 = np.zeros((b, max(L, 4), 2), np.float32)
+    lm4[:, :L] = lm
+    sb.prime(layout(0))
+    try:
+        for f in (1, 2):
+            out = {k: np.array(v) for k, v in sb.step(layout(f), lm4, obj, n_pts, cand, n_cand).items()}
+            for k, (r, c) in enumerate(sizes):
+                for name, p in (("lm", pts[k]), ("cand", cand_of[k])):
+                    if not len(p):
+                        continue
+                    rp, rst, _ = oracle.calc_optical_flow_pyr_lk(crops[k][f - 1], crops[k][f], p, win, ml, crit)
+                    st, nxt = out[name + "_status"][k, :len(p)], out[name + "_next"][k, :len(p)]
+                    ok = rst.ravel() == 1
+                    if not (np.array_equal(st, rst.ravel()) and np.array_equal(nxt[ok], rp[ok])):
+                        bad.append(("batch-klt", slot, (r, c), win, ml, crit, f, name, int((st != rst.ravel()).sum())))
+                    stats["batch_klt"] += 1
+        mc = int(rng.choice([1, 7, 50, 1400, 5000]))
+        q = float(rng.choice([0.1, 0.03, 0.01, 0.3]))
+        md = float(rng.choice([1, 2, 3, 5, 7.5, 10, 25]))
+        cell = int(np.rint(md))
+        if -(-slot[0] // cell) * -(-slot[1] // cell) * 16 > 200 * 1024:
+            md = float(rng.choice([10, 25]))
+        try:
+            corners, nc = sb.good_features(mc, q, md)
+        except _lib.B200VOError as e:
+            if "exceed" not in str(e):      # more candidates than the batched path ranks: refused, not wrong
+                raise
+            return
+        for k in range(b):
+            want = oracle.good_features_to_track(crops[k][2], mc, q, md)
+            want = np.zeros((0, 2), np.float32) if want is None else want.reshape(-1, 2)
+            if nc[k] != len(want) or not np.array_equal(corners[k, :nc[k]], want):
+                bad.append(("batch-gftt", slot, sizes[k], mc, q, md, int(nc[k]), len(want)))
+            stats["batch_gftt"] += 1
+    finally:
+        sb.close()
 
 
 def main():
     budget = float(sys.argv[1]) if len(sys.argv) > 1 else 120.0
     rng = np.random.default_rng(int(os.environ.get("FUZZ_SEED", "1")))
     t_end = time.time() + budget
-    stats = dict(klt=0, gftt=0, knn=0, pnp=0, emat=0, rpose=0, mind=0, tri=0, sift=0)
+    stats = dict(klt=0, gftt=0, knn=0, pnp=0, emat=0, rpose=0, mind=0, tri=0, sift=0, batch=0, batch_klt=0, batch_gftt=0)
     bad = []
+    # FUZZ_KINDS=batch: only the batch kind
+    only_batch = os.environ.get("FUZZ_KINDS", "") == "batch"
 
     def rand_frames():
         shape = str(rng.choice(["kitti", "parking", "malaga"]))
@@ -41,9 +139,12 @@ def main():
     it = 0
     while time.time() < t_end:
         it += 1
-        kind = it % 9
+        kind = 9 if only_batch else it % 10
         try:
-            if kind in (0, 1, 2):
+            if kind == 9:
+                batch_case(rng, bad, stats)
+                stats["batch"] += 1
+            elif kind in (0, 1, 2):
                 f0, f1 = rand_frames()["frames"]
                 h, w = f0.shape
                 win = [(15, 15), (21, 21), (9, 13), (31, 31), (5, 7), (21, 15)][int(rng.integers(0, 6))]
