@@ -406,6 +406,33 @@ int b200vo_loop_step(b200vo_loop* lp, const uint8_t* frames, int32_t* status, in
 /* The same with device pointers; asynchronous on the ctx stream (never synchronises the host). */
 int b200vo_loop_step_dev(b200vo_loop* lp, const uint8_t* frames_dev, int32_t* status_dev, int32_t* n_inliers_dev,
                          int32_t* n_lm_dev, int32_t* n_cand_dev, double* pose_cw_dev);
+/* Listed steps: a step that advances only the n_seq distinct sequences seqs[] (any order), for streams that do not tick
+ * together (different lengths or frame rates, dropped frames).  frames: uint8 [n_seq][rows][cols] in the slot layout and
+ * in list order (only these are uploaded); NULL: the oldest submitted set, which must have been submitted with the same
+ * list by b200vo_loop_submit_frames_seqs(_dev).  Full and listed sets may alternate in the FIFO and are consumed in order;
+ * b200vo_loop_step(NULL) refuses a listed set and a listed step a full one.
+ * A listed sequence runs exactly the step it runs in a batch of one, bit for bit (nothing in a step depends on how many
+ * steps the batch has taken), so its results and state depend only on its own frames and the calls that list it.  A
+ * sequence that is not listed is not touched: its state, status and current frame stay as they are, and its next listed
+ * step tracks from that frame.  A listed sequence that is not B200VO_LOOP_OK is reported as b200vo_loop_step reports it.
+ * Results: n_seq rows in list order (status, n_inliers, n_lm, n_cand int32 [n_seq], pose_cw double [n_seq][12]).
+ * seqs is a HOST array in all four calls, the _dev forms included: the call validates it and sizes its launches from
+ * it; the library keeps its own copy, so the caller may reuse it as soon as the call returns.
+ * B200VO_E_BADARG, before any device work and with nothing changed: n_seq < 1 or > batch, an index out of range or
+ * repeated, a null array, frames == NULL with nothing submitted or with a set submitted with another list (or with none),
+ * frames passed while submitted sets are waiting.
+ * b200vo_loop_step_seqs synchronises as b200vo_loop_step (one upload of the listed frames, one read-back of n_seq rows);
+ * the _dev forms never synchronise the host.  The pyramids, the detector and the loop kernels work for the listed
+ * sequences only, the trackers and the pose chain see a count of 0 for the others, and every other sequence's current
+ * pyramid is copied into the step's pyramid set. */
+int b200vo_loop_step_seqs(b200vo_loop* lp, int n_seq, const int32_t* seqs, const uint8_t* frames, int32_t* status,
+                          int32_t* n_inliers, int32_t* n_lm, int32_t* n_cand, double* pose_cw);
+int b200vo_loop_step_seqs_dev(b200vo_loop* lp, int n_seq, const int32_t* seqs, const uint8_t* frames_dev, int32_t* status_dev,
+                              int32_t* n_inliers_dev, int32_t* n_lm_dev, int32_t* n_cand_dev, double* pose_cw_dev);
+/* Frames of a future listed step: uint8 [n_seq][rows][cols] (page-locked host memory, or device memory for _dev) for
+ * the sequences seqs[] (host array), as b200vo_loop_submit_frames(_dev).  Same list validation. */
+int b200vo_loop_submit_frames_seqs(b200vo_loop* lp, int n_seq, const int32_t* seqs, const uint8_t* frames);
+int b200vo_loop_submit_frames_seqs_dev(b200vo_loop* lp, int n_seq, const int32_t* seqs, const uint8_t* frames_dev);
 
 int b200vo_sync(b200vo_ctx* ctx);
 /* Page-locked host memory for frame buffers: b200vo_batch_step DMAs straight out of such a

@@ -128,6 +128,10 @@ SIGNATURES = {
     "b200vo_loop_submit_frames_dev": (C.c_int, [C.c_void_p, C.c_void_p]),
     "b200vo_loop_step": (C.c_int, [C.c_void_p, c_u8p, c_i32p, c_i32p, c_i32p, c_i32p, c_f64p]),
     "b200vo_loop_step_dev": (C.c_int, [C.c_void_p] + [C.c_void_p] * 6),
+    "b200vo_loop_step_seqs": (C.c_int, [C.c_void_p, C.c_int, c_i32p, c_u8p, c_i32p, c_i32p, c_i32p, c_i32p, c_f64p]),
+    "b200vo_loop_step_seqs_dev": (C.c_int, [C.c_void_p, C.c_int, c_i32p] + [C.c_void_p] * 6),
+    "b200vo_loop_submit_frames_seqs": (C.c_int, [C.c_void_p, C.c_int, c_i32p, c_u8p]),
+    "b200vo_loop_submit_frames_seqs_dev": (C.c_int, [C.c_void_p, C.c_int, c_i32p, C.c_void_p]),
     "b200vo_sync": (C.c_int, [C.c_void_p]),
     "b200vo_host_alloc": (C.c_void_p, [C.c_void_p, C.c_size_t]),
     "b200vo_host_free": (None, [C.c_void_p, C.c_void_p]),

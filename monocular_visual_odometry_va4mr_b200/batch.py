@@ -461,24 +461,73 @@ class VOBatch:
         return dict(lm=lm[:nl], lm_kp=kp[:nl], keys=keys[:nc], first_keys=fk[:nc], first_pose=fp[:nc], poses=poses[:npo],
                     status=status.value)
 
-    def submit_frames(self, frames):
+    def _list(self, seqs) -> np.ndarray:
+        """The sequences of a listed step as int32 (n,); ValueError unless they are 1 to batch distinct indices in [0, batch)."""
+        a = np.asarray(seqs)
+        if a.ndim != 1 or a.size < 1 or a.size > self.batch or not np.issubdtype(a.dtype, np.integer):
+            raise ValueError(f"seqs must be 1 to batch = {self.batch} integer sequence indices, got {a.dtype} {a.shape}")
+        if ((a < 0) | (a >= self.batch)).any():
+            raise ValueError(f"seqs must lie in [0, batch = {self.batch})")
+        if len(np.unique(a)) != len(a):
+            raise ValueError("seqs must be distinct")
+        return np.ascontiguousarray(a, np.int32)
+
+    def _listed_frames(self, frames, seqs, out=None) -> np.ndarray:
+        """frames of a listed step: (len(seqs), rows, cols) uint8 in the slot layout, or a list of the listed sequences' images"""
+        frames = _pack_frames(frames, self.frame_size[seqs], self.rows, self.cols, out)
+        if not isinstance(frames, np.ndarray) or frames.dtype != np.uint8 or frames.shape != (len(seqs), self.rows, self.cols):
+            raise ValueError(f"frames must be ({len(seqs)}, {self.rows}, {self.cols}) uint8 or a list of {len(seqs)} images")
+        return np.ascontiguousarray(frames)
+
+    def submit_frames(self, frames, seqs=None):
         """Frames of a FUTURE step (page-locked, from pinned_frames(), or a list of per-sequence images, packed into a page-locked
-        copy); step(None) consumes them, oldest first."""
+        copy); step(None) consumes them, oldest first.  ``seqs``: the frames of a listed step (see ``step``), consumed by
+        ``step(None, seqs)`` with the same list."""
+        if seqs is not None:
+            seqs = self._list(seqs)
+            if isinstance(frames, (list, tuple)):
+                frames = self._listed_frames(frames, seqs, self.pinned_empty((len(seqs), self.rows, self.cols), np.uint8))
+                self._submitted = (self._submitted + [frames])[-3:]
+            else:
+                frames = self._listed_frames(frames, seqs)
+            self._chk(self.ctx.lib.b200vo_loop_submit_frames_seqs(self.h, len(seqs), _p(seqs, c_i32p), _p(frames, c_u8p)),
+                      "b200vo_loop_submit_frames_seqs")
+            return
         if isinstance(frames, (list, tuple)):
             frames = _pack_frames(frames, self.frame_size, self.rows, self.cols, self.pinned_frames()[0])
             self._submitted = (self._submitted + [frames])[-3:]
         assert frames.dtype == np.uint8 and frames.flags.c_contiguous and frames.size == self.batch * self.rows * self.cols
         self._chk(self.ctx.lib.b200vo_loop_submit_frames(self.h, _p(frames, c_u8p)), "b200vo_loop_submit_frames")
 
-    def submit_frames_dev(self, frames_dev: int):
-        """The same for frames resident in device memory (int from tensor.data_ptr()); step_dev(None, ...) consumes them."""
+    def submit_frames_dev(self, frames_dev: int, seqs=None):
+        """The same for frames resident in device memory (int from tensor.data_ptr()); step_dev(None, ...) consumes them.
+        ``seqs``: (len(seqs), rows, cols) frames of a listed step, consumed by ``step_dev(None, out_dev, seqs)``."""
+        if seqs is not None:
+            seqs = self._list(seqs)
+            self._chk(self.ctx.lib.b200vo_loop_submit_frames_seqs_dev(self.h, len(seqs), _p(seqs, c_i32p), frames_dev),
+                      "b200vo_loop_submit_frames_seqs_dev")
+            return
         self._chk(self.ctx.lib.b200vo_loop_submit_frames_dev(self.h, frames_dev), "b200vo_loop_submit_frames_dev")
 
-    def step(self, frames=None) -> dict:
+    def step(self, frames=None, seqs=None) -> dict:
         """One frame for every sequence (frames (batch, rows, cols) uint8 in the slot layout, or a list of per-sequence images;
         None: the oldest submitted set).  Synchronous.
         Returns views on REUSED page-locked arrays: status, n_inliers, n_lm, n_cand int32 (batch,) and pose_cw float64
-        (batch, 12), the pose appended this step (0 unless status is OK)."""
+        (batch, 12), the pose appended this step (0 unless status is OK).
+
+        ``seqs``: a listed step that advances only the distinct sequences ``seqs`` (any order), e.g. the streams that have a
+        new frame this tick.  frames are then (len(seqs), rows, cols) or a list of the listed sequences' images, in list
+        order; None consumes a set submitted with the same list.  Each listed sequence runs exactly the step it runs in a
+        batch of its own; the others are not touched and resume from their current frame when they are listed again.  The
+        results are the first len(seqs) rows of the same arrays, in list order.  Bad shapes or indices raise ValueError."""
+        if seqs is not None:
+            seqs = self._list(seqs)
+            n = len(seqs)
+            if frames is not None:
+                frames = self._listed_frames(frames, seqs)
+            self._chk(self.ctx.lib.b200vo_loop_step_seqs(self.h, n, _p(seqs, c_i32p), _p(frames, c_u8p) if frames is not None else None,
+                                                         *self._res_ptrs), "b200vo_loop_step_seqs")
+            return {k: v[:n] for k, v in self._res.items()}
         if frames is not None:
             frames = np.ascontiguousarray(_pack_frames(frames, self.frame_size, self.rows, self.cols), np.uint8)
             assert frames.size == self.batch * self.rows * self.cols
@@ -486,11 +535,18 @@ class VOBatch:
                   "b200vo_loop_step")
         return self._res
 
-    def step_dev(self, frames_dev, out_dev: dict):
+    def step_dev(self, frames_dev, out_dev: dict, seqs=None):
         """Device pointers (ints from tensor.data_ptr()) for the frames (None: the oldest submitted set) and for the results
         ``status``, ``n_inliers``, ``n_lm``, ``n_cand`` (int32 (batch,)) and ``pose_cw`` (float64 (batch, 12)).
-        Asynchronous on the ctx stream."""
+        Asynchronous on the ctx stream.  ``seqs``: a listed step (see ``step``): frames_dev holds (len(seqs), rows, cols),
+        and the results fill the first len(seqs) rows in list order."""
         o = out_dev
+        if seqs is not None:
+            seqs = self._list(seqs)
+            self._chk(self.ctx.lib.b200vo_loop_step_seqs_dev(self.h, len(seqs), _p(seqs, c_i32p), frames_dev or None, o['status'],
+                                                             o['n_inliers'], o['n_lm'], o['n_cand'], o['pose_cw']),
+                      "b200vo_loop_step_seqs_dev")
+            return
         self._chk(self.ctx.lib.b200vo_loop_step_dev(self.h, frames_dev or None, o['status'], o['n_inliers'], o['n_lm'], o['n_cand'],
                                                     o['pose_cw']), "b200vo_loop_step_dev")
 

@@ -255,7 +255,8 @@ extern "C" void b200vo_batch_destroy(b200vo_batch* B)
     kill_stream(B->io_stream);
     kill_stream(B->pose_stream);
     for (auto& s : B->slabs) if (s.p) cudaFree(s.p);
-    for (DevBuf* d : {&B->raw, &B->raw_pre, &B->pts_in, &B->outs, &B->work, &B->gftt_ws, &B->intr_buf, &B->ext_buf}) if (d->p) cudaFree(d->p);
+    for (DevBuf* d : {&B->raw, &B->raw_pre, &B->pts_in, &B->outs, &B->work, &B->gftt_ws, &B->intr_buf, &B->ext_buf, &B->lists})
+        if (d->p) cudaFree(d->p);
     for (auto& e : B->q_ev) kill_event(e);
     for (auto& e : B->chunk_ev) kill_event(e);
     for (auto& e : B->copy_ev) kill_event(e);
@@ -297,9 +298,21 @@ int batch_free_set(const b200vo_batch* B)
     return -1;
 }
 
+// the device row of a list: [list | pos], see b200vo_batch::lists
+static int* batch_list_row(const b200vo_batch* B, int row) { return (int*)B->lists.p + (size_t)row * 2 * B->batch; }
+
+// upload a list into its device row on `stream` (a pageable source: staged before the call returns, nothing waits)
+static int batch_upload_list(b200vo_batch* B, int row, int n, const int32_t* list, cudaStream_t stream)
+{
+    std::vector<int32_t> r(2 * (size_t)B->batch, -1);
+    for (int k = 0; k < n; ++k) { r[k] = list[k]; r[B->batch + list[k]] = k; }
+    VO_CUDA(B->ctx, cudaMemcpyAsync(batch_list_row(B, row), r.data(), r.size() * 4, cudaMemcpyHostToDevice, stream));
+    return 0;
+}
+
 // Frames of a FUTURE step: copied and turned into pyramids on a side stream while the current step's
 // kernels run; the step that passes frames == NULL consumes them (oldest first).
-int batch_submit(b200vo_batch* B, const uint8_t* frames, bool dev)
+int batch_submit(b200vo_batch* B, const uint8_t* frames, bool dev, int n_list, const int32_t* list)
 {
     if (!B || !frames) return B200VO_E_BADARG;
     b200vo_ctx* ctx = B->ctx;
@@ -324,6 +337,7 @@ int batch_submit(b200vo_batch* B, const uint8_t* frames, bool dev)
     B->q_set[slot] = set;
     B->q_src[slot] = frames;
     B->q_dev[slot] = dev;
+    B->q_list[slot].assign(list, list + n_list);
     B->q_count++;
     return 0;
 }
@@ -349,14 +363,24 @@ int batch_issue_prefetch(b200vo_batch* B, cudaEvent_t after, bool wait_step_end)
         if (!B->q_src[slot]) continue;
         if (wait_step_end) VO_CUDA(ctx, cudaStreamWaitEvent(B->pre_stream, B->step_end_ev, 0));   // readers of this set have retired
         if (after) VO_CUDA(ctx, cudaStreamWaitEvent(B->pre_stream, after, 0));  // and the step's own uploads have landed
+        const std::vector<int32_t>& ql = B->q_list[slot];
+        // a listed set: its list row was last read by the step that consumed the slot's previous set, which ended before
+        // step_end_ev (the pyramid build of this slot is issued by a later call)
+        if (!ql.empty()) VO_TRY(batch_upload_list(B, slot, (int)ql.size(), ql.data(), B->pre_stream));
         const uint8_t* raw = B->q_src[slot];
         if (!B->q_dev[slot]) {
-            VO_CUDA(ctx, cudaMemcpyAsync(B->raw_pre.p, B->q_src[slot], total, cudaMemcpyHostToDevice, B->pre_stream));
+            VO_CUDA(ctx, cudaMemcpyAsync(B->raw_pre.p, B->q_src[slot], ql.empty() ? total : fb * ql.size(), cudaMemcpyHostToDevice,
+                                         B->pre_stream));
             raw = (const uint8_t*)B->raw_pre.p;
         }
-        VO_TRY(vo_build_pyramids(ctx, raw, fb, B->cfg.rows, B->cfg.cols, B->geom,
-                                 (uint8_t*)B->slabs[B->q_set[slot]].p, B->geom.slab_bytes, B->batch, B->pre_stream, batch_ext_dev(B, 0),
-                                 batch_ext_host(B, 0)));
+        if (ql.empty())
+            VO_TRY(vo_build_pyramids(ctx, raw, fb, B->cfg.rows, B->cfg.cols, B->geom,
+                                     (uint8_t*)B->slabs[B->q_set[slot]].p, B->geom.slab_bytes, B->batch, B->pre_stream, batch_ext_dev(B, 0),
+                                     batch_ext_host(B, 0)));
+        else
+            VO_TRY(vo_build_pyramids(ctx, raw, fb, B->cfg.rows, B->cfg.cols, B->geom, (uint8_t*)B->slabs[B->q_set[slot]].p,
+                                     B->geom.slab_bytes, (int)ql.size(), B->pre_stream, batch_ext_dev(B, 0), batch_ext_host(B, 0), 0,
+                                     batch_list_row(B, slot), ql.data(), B->batch));
         VO_CUDA(ctx, cudaEventRecord(B->q_ev[slot], B->pre_stream));
         B->q_src[slot] = nullptr;
     }
@@ -394,7 +418,10 @@ static int batch_track(b200vo_batch* B, cudaStream_t stream, int b0, int nb, con
     if (which == 0 || which == 3 || which == 4) {
         const bool whole = b0 == 0 && nb == B->batch;   // chunked uploads build the pyramids piecewise: no single interval to time
         if (whole) prof_mark(B, 0, stream);
-        if (frames_dev)
+        if (frames_dev && B->step_list)   // the listed images into their sequences' slabs (b0 == 0, nb == batch)
+            VO_TRY(vo_build_pyramids(ctx, frames_dev, fb, c.rows, c.cols, B->geom, (uint8_t*)B->slabs[nxt].p, sb, B->step_n, stream,
+                                     batch_ext_dev(B, 0), batch_ext_host(B, 0), 0, B->step_list, B->step_list_host, B->batch));
+        else if (frames_dev)
             VO_TRY(vo_build_pyramids(ctx, frames_dev + (size_t)b0 * fb, fb, c.rows, c.cols, B->geom,
                                      (uint8_t*)B->slabs[nxt].p + (size_t)b0 * sb, sb, nb, stream, batch_ext_dev(B, b0), batch_ext_host(B, b0)));
         if (whole) { prof_mark(B, 1, stream); B->prof_row_open = B->profile && B->prof_n < B200VO_PROF_RING; }
@@ -460,6 +487,7 @@ int batch_finish(b200vo_batch* B)
 {
     VO_CUDA(B->ctx, cudaEventRecord(B->step_end_ev, B->ctx->stream));
     B->cur = B->nxt;
+    B->step_list = nullptr; B->step_list_host = nullptr; B->step_n = 0;
     return 0;
 }
 
@@ -500,9 +528,10 @@ int batch_track_pose_overlapped(b200vo_batch* B, const uint8_t* frames_dev, cons
     return 0;
 }
 
-int batch_select_frames(b200vo_batch* B, const uint8_t* frames_dev)
+int batch_select_frames(b200vo_batch* B, const uint8_t* frames_dev, int n_list, const int32_t* list)
 {
     b200vo_ctx* ctx = B->ctx;
+    B->step_list = nullptr; B->step_list_host = nullptr; B->step_n = 0;
     if (!frames_dev) {
         // the frames were handed over by b200vo_batch_submit_frames(_dev): their pyramids were (or are being) built on
         // the side stream, beside the previous step
@@ -510,6 +539,7 @@ int batch_select_frames(b200vo_batch* B, const uint8_t* frames_dev)
             return vo_set_err(ctx, B200VO_E_BADARG, "frames == NULL but no frame set was submitted (b200vo_batch_submit_frames[_dev])");
         const int q_slot = B->q_head;
         VO_TRY(batch_issue_prefetch(B));                     // whatever is still waiting, this step's set first
+        if (n_list > 0) { B->step_list = batch_list_row(B, q_slot); B->step_list_host = B->q_list[q_slot].data(); B->step_n = n_list; }
         B->nxt = B->q_set[q_slot];
         B->q_head ^= 1;
         B->q_count--;
@@ -520,6 +550,10 @@ int batch_select_frames(b200vo_batch* B, const uint8_t* frames_dev)
         const int free_set = batch_free_set(B);
         if (free_set < 0) return vo_set_err(ctx, B200VO_E_BADARG, "no free pyramid set");
         B->nxt = free_set;
+        if (n_list > 0) {   // row 2: the previous step that read it is ordered before this upload on the ctx stream
+            VO_TRY(batch_upload_list(B, 2, n_list, list, ctx->stream));
+            B->step_list = batch_list_row(B, 2); B->step_list_host = list; B->step_n = n_list;
+        }
     }
     return 0;
 }

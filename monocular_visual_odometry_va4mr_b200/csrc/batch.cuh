@@ -22,6 +22,15 @@ struct b200vo_batch {
     int q_set[2]; int q_head = 0, q_count = 0;
     const uint8_t* q_src[2] = {};   // frames whose copy / pyramid build has not been enqueued yet (see batch_issue_prefetch)
     bool q_dev[2] = {};             // q_src is device memory (b200vo_batch_submit_frames_dev): no copy, pyramids straight from it
+    // Listed steps (b200vo_loop_step_seqs): a submitted set or a step's frames may cover only the sequences of a list.  Each
+    // list lives on the device as a row of 2 * batch ints, [list (n entries) | pos (batch entries: row in the list or -1)]:
+    // row 0 / 1 belongs to FIFO slot 0 / 1 (uploaded on the side stream when the set's pyramids are enqueued, after the
+    // step that last read the row has ended), row 2 to a step that passes its frames (uploaded on the ctx stream).
+    std::vector<int32_t> q_list[2]; // the list a submitted set was given; empty: a full set
+    DevBuf lists;                   // [3][2 * batch] int32
+    const int* step_list = nullptr; // the device row of the step being enqueued; nullptr: every sequence
+    const int32_t* step_list_host = nullptr;
+    int step_n = 0;                 // its length
     cudaEvent_t q_ev[2] = {};
     cudaStream_t pre_stream = nullptr;
     cudaEvent_t step_end_ev = nullptr;
@@ -74,8 +83,11 @@ struct b200vo_batch {
 
 // the frames of the step about to be enqueued: a submitted set (frames_dev == nullptr) or a free set the step builds
 // its pyramids in; sets B->nxt and makes the ctx stream wait for a prefetched set
-int batch_select_frames(b200vo_batch* B, const uint8_t* frames_dev);
-int batch_submit(b200vo_batch* B, const uint8_t* frames, bool dev);
+// With n_list > 0 the step covers the sequences list[0 .. n_list) only (validated by the caller): frames_dev holds their
+// images in list order, or the oldest submitted set was submitted with that list; sets step_list / step_n.
+int batch_select_frames(b200vo_batch* B, const uint8_t* frames_dev, int n_list = 0, const int32_t* list = nullptr);
+// a frame set for a later step; n_list > 0: the images of the sequences list[0 .. n_list) in list order (validated by the caller)
+int batch_submit(b200vo_batch* B, const uint8_t* frames, bool dev, int n_list = 0, const int32_t* list = nullptr);
 int batch_issue_prefetch(b200vo_batch* B, cudaEvent_t after = nullptr, bool wait_step_end = true);
 int batch_free_set(const b200vo_batch* B);
 int batch_track_pose_overlapped(b200vo_batch* B, const uint8_t* frames_dev, const float* lm_pts, const float* lm_obj,

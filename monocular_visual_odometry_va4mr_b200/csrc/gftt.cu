@@ -160,14 +160,16 @@ gftt_colsum_kernel(const float* __restrict__ cov, int w, int h, float* __restric
 #define GF_COLS 30
 __global__ void __launch_bounds__(32)
 gftt_fused_eig_kernel(const uint8_t* __restrict__ img, size_t img_stride, int pitch, int w, int h, float k0, float k1,
-                      float* __restrict__ eig, int* __restrict__ max_bits, int small_stride, const VoSeqExt* __restrict__ ext)
+                      float* __restrict__ eig, int* __restrict__ max_bits, int small_stride, const VoSeqExt* __restrict__ ext,
+                      const int* __restrict__ list)
 {
     const int lane = threadIdx.x;
-    img += blockIdx.y * img_stride;
-    eig += (size_t)blockIdx.y * w * h;          // planes of the slot size; a sequence's own plane has rows of its own width
-    max_bits += blockIdx.y * small_stride;
+    const int im = list ? list[blockIdx.y] : blockIdx.y;
+    img += im * img_stride;
+    eig += (size_t)im * w * h;                  // planes of the slot size; a sequence's own plane has rows of its own width
+    max_bits += im * small_stride;
     if (ext) {
-        w = ext[blockIdx.y].w[0]; h = ext[blockIdx.y].h[0];
+        w = ext[im].w[0]; h = ext[im].h[0];
         if ((int)blockIdx.x * GF_COLS >= w) return;
     }
     const int xv = blockIdx.x * GF_COLS + lane - 1;            // virtual column (may be -1 or >= w)
@@ -320,13 +322,14 @@ gftt_eig_kernel(const float* __restrict__ box, int w, int h, float* __restrict__
 __global__ void __launch_bounds__(256)
 gftt_candidates_kernel(const float* __restrict__ eig, int w, int h, const int* __restrict__ max_bits, double quality,
                        unsigned long long* __restrict__ keys, int* __restrict__ n_keys, int cap, int small_stride,
-                       const VoSeqExt* __restrict__ ext = nullptr)
+                       const VoSeqExt* __restrict__ ext = nullptr, const int* __restrict__ list = nullptr)
 {
-    eig += (size_t)blockIdx.z * w * h;
-    if (ext) { w = ext[blockIdx.z].w[0]; h = ext[blockIdx.z].h[0]; }   // key address y * w + x: cv2's tie order in its own image
-    max_bits += blockIdx.z * small_stride;
-    n_keys += blockIdx.z * small_stride;
-    keys += (size_t)blockIdx.z * cap;
+    const int im = list ? list[blockIdx.z] : blockIdx.z;
+    eig += (size_t)im * w * h;
+    if (ext) { w = ext[im].w[0]; h = ext[im].h[0]; }   // key address y * w + x: cv2's tie order in its own image
+    max_bits += im * small_stride;
+    n_keys += im * small_stride;
+    keys += (size_t)im * cap;
     const int x = blockIdx.x * blockDim.x + threadIdx.x + 1;
     const float thr = (float)((double)__int_as_float(*max_bits) * quality);
     const int lane = (threadIdx.y * blockDim.x + threadIdx.x) & 31;
@@ -356,12 +359,13 @@ gftt_candidates_kernel(const float* __restrict__ eig, int w, int h, const int* _
 // descending order of the 64-bit keys = (value desc, address desc); keys are unique
 __global__ void __launch_bounds__(256)
 gftt_rank_kernel(const unsigned long long* __restrict__ keys, const int* __restrict__ n_keys, int cap,
-                 unsigned long long* __restrict__ sorted, int small_stride)
+                 unsigned long long* __restrict__ sorted, int small_stride, const int* __restrict__ list = nullptr)
 {
     __shared__ unsigned long long tile[1024];
-    keys += (size_t)blockIdx.y * cap;
-    sorted += (size_t)blockIdx.y * cap;
-    n_keys += blockIdx.y * small_stride;
+    const int im = list ? list[blockIdx.y] : blockIdx.y;
+    keys += (size_t)im * cap;
+    sorted += (size_t)im * cap;
+    n_keys += im * small_stride;
     const int n = min(*n_keys, cap);
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (blockIdx.x * blockDim.x >= n) return;
@@ -471,17 +475,19 @@ gftt_select_kernel(const unsigned long long* __restrict__ sorted, const int* __r
 __global__ void __launch_bounds__(256)
 gftt_select_smem_kernel(const unsigned long long* __restrict__ sorted, const int* __restrict__ n_keys, int cap, int w, int h,
                         int max_corners, double min_dist, int cell, int gw, int gh, float* __restrict__ corners,
-                        int* __restrict__ n_out, int small_stride, size_t out_stride, const VoSeqExt* __restrict__ ext = nullptr)
+                        int* __restrict__ n_out, int small_stride, size_t out_stride, const VoSeqExt* __restrict__ ext = nullptr,
+                        const int* __restrict__ list = nullptr)
 {
     extern __shared__ uint4 s_cells[];
+    const int im = list ? list[blockIdx.x] : blockIdx.x;   // one CTA per image
     if (ext) {   // the image's own cell grid (the shared memory is sized for the slot's)
-        w = ext[blockIdx.x].w[0]; h = ext[blockIdx.x].h[0];
+        w = ext[im].w[0]; h = ext[im].h[0];
         gw = (w + cell - 1) / cell; gh = (h + cell - 1) / cell;
     }
-    sorted += (size_t)blockIdx.x * cap;                   // one CTA per image
-    n_keys += blockIdx.x * small_stride;
-    n_out += blockIdx.x * small_stride;
-    corners += blockIdx.x * out_stride;
+    sorted += (size_t)im * cap;
+    n_keys += im * small_stride;
+    n_out += im * small_stride;
+    corners += im * out_stride;
     for (int i = threadIdx.x; i < gw * gh; i += blockDim.x) s_cells[i] = make_uint4(~0u, ~0u, ~0u, ~0u);
     __syncthreads();
     if (threadIdx.x >= 32) return;
@@ -683,9 +689,10 @@ size_t vo_gftt_batch_workspace(int rows, int cols, int batch, int max_corners)
 
 int vo_gftt_batch_launch(b200vo_ctx* ctx, const uint8_t* d_img0, size_t img_stride, int pitch, int rows, int cols, int batch,
                          int max_corners, double quality, double min_dist, void* ws, float** d_corners_out, int** d_small_out,
-                         const VoSeqExt* d_ext)
+                         const VoSeqExt* d_ext, const int* d_list, int n_img)
 {
     const int w = cols, h = rows;
+    if (!d_list) n_img = batch;
     const size_t npx = (size_t)w * h;
     if (!(quality > 0) || min_dist < 0 || max_corners < 0)
         return vo_set_err(ctx, B200VO_E_BADARG, "qualityLevel > 0 && minDistance >= 0 && maxCorners >= 0");
@@ -705,15 +712,18 @@ int vo_gftt_batch_launch(b200vo_ctx* ctx, const uint8_t* d_img0, size_t img_stri
     VO_CUDA(ctx, cudaMemsetAsync(d_small, 0, (size_t)batch * GFTT_SMALL * sizeof(int), ctx->stream));
     const double scale = 1.0 / (4.0 * 3 * 255.0);
     dim3 blk(32, 8);
-    gftt_fused_eig_kernel<<<dim3((w + GF_COLS - 1) / GF_COLS, batch), 32, 0, ctx->stream>>>(d_img0, img_stride, pitch, w, h, (float)scale,
-                                                                                            (float)(2.0 * scale), d_eig, d_small, GFTT_SMALL, d_ext);
-    gftt_candidates_kernel<<<dim3((w - 2 + 31) / 32, (h - 2 + 31) / 32, batch), blk, 0, ctx->stream>>>(d_eig, w, h, d_small, quality, d_keys,
-                                                                                                    d_small + 1, GFTT_BATCH_CAP, GFTT_SMALL, d_ext);
-    gftt_rank_kernel<<<dim3(GFTT_BATCH_CAP / 256, batch), 256, 0, ctx->stream>>>(d_keys, d_small + 1, GFTT_BATCH_CAP, d_sorted, GFTT_SMALL);
+    gftt_fused_eig_kernel<<<dim3((w + GF_COLS - 1) / GF_COLS, n_img), 32, 0, ctx->stream>>>(d_img0, img_stride, pitch, w, h, (float)scale,
+                                                                                            (float)(2.0 * scale), d_eig, d_small, GFTT_SMALL, d_ext,
+                                                                                            d_list);
+    gftt_candidates_kernel<<<dim3((w - 2 + 31) / 32, (h - 2 + 31) / 32, n_img), blk, 0, ctx->stream>>>(d_eig, w, h, d_small, quality, d_keys,
+                                                                                                    d_small + 1, GFTT_BATCH_CAP, GFTT_SMALL, d_ext,
+                                                                                                    d_list);
+    gftt_rank_kernel<<<dim3(GFTT_BATCH_CAP / 256, n_img), 256, 0, ctx->stream>>>(d_keys, d_small + 1, GFTT_BATCH_CAP, d_sorted, GFTT_SMALL,
+                                                                                 d_list);
     if (cell_smem > 48 * 1024)
         VO_CUDA(ctx, cudaFuncSetAttribute(gftt_select_smem_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cell_smem));
-    gftt_select_smem_kernel<<<batch, 256, cell_smem, ctx->stream>>>(d_sorted, d_small + 1, GFTT_BATCH_CAP, w, h, max_corners, min_dist, cell,
-                                                                    gw, gh, d_out, d_small + 2, GFTT_SMALL, b_out / 4, d_ext);
+    gftt_select_smem_kernel<<<n_img, 256, cell_smem, ctx->stream>>>(d_sorted, d_small + 1, GFTT_BATCH_CAP, w, h, max_corners, min_dist, cell,
+                                                                    gw, gh, d_out, d_small + 2, GFTT_SMALL, b_out / 4, d_ext, d_list);
     ctx->launches += 4;
     VO_CUDA(ctx, cudaGetLastError());
     *d_corners_out = d_out;

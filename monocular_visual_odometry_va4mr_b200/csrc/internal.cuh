@@ -168,18 +168,22 @@ void vo_seq_ext(int rows, int cols, int win_w, int win_h, int max_level, VoSeqEx
 // raw (device, rows of `raw_row` bytes, 0: cols) -> bordered level 0, then levels 1..L-1; `batch` slabs/raws strided.
 // d_ext / h_ext: [batch] per-sequence extents on the device and their host copy (both or neither), each inside the
 // slot geometry g; every level of a sequence is built at its own size, levels beyond its own count are not built.
+// d_list / h_list (both or neither): raw image k goes to slab list[k] of the n_slab slabs at d_slab, with the extents
+// ext[list[k]] (the tables then cover all n_slab slabs); the other slabs are not touched.
 int vo_build_pyramids(b200vo_ctx* ctx, const uint8_t* d_raw, size_t raw_stride, int rows, int cols,
                       const PyrGeom& g, uint8_t* d_slab, size_t slab_stride, int batch, cudaStream_t stream,
-                      const VoSeqExt* d_ext = nullptr, const VoSeqExt* h_ext = nullptr, size_t raw_row = 0);
+                      const VoSeqExt* d_ext = nullptr, const VoSeqExt* h_ext = nullptr, size_t raw_row = 0,
+                      const int* d_list = nullptr, const int* h_list = nullptr, int n_slab = 0);
 
 // ---- gftt.cu: detection on device-resident bordered level-0 images, one per batch entry ----
 #define VO_GFTT_SMALL 4          // ints per image in the result block: max bits | n candidates | n corners | spare
 #define VO_GFTT_BATCH_CAP 32768  // candidates per image the batched path can rank
 size_t vo_gftt_batch_workspace(int rows, int cols, int batch, int max_corners);
-// d_ext: [batch] per-sequence extents (level 0 is read), nullptr: every image is rows x cols
+// d_ext: [batch] per-sequence extents (level 0 is read), nullptr: every image is rows x cols.  d_list: only the n_img
+// images list[k] are detected; their outputs keep the image index (the others' are left stale)
 int vo_gftt_batch_launch(b200vo_ctx* ctx, const uint8_t* d_img0, size_t img_stride, int pitch, int rows, int cols, int batch,
                          int max_corners, double quality, double min_dist, void* ws, float** d_corners_out, int** d_small_out,
-                         const VoSeqExt* d_ext = nullptr);
+                         const VoSeqExt* d_ext = nullptr, const int* d_list = nullptr, int n_img = 0);
 
 // ---- klt.cu ----
 struct KltPointSet {

@@ -21,8 +21,10 @@
 #include "sift.cuh"
 #include "mathdev.cuh"
 #include "pnp.cuh"
+#include <algorithm>
 
 #define LOOP_T 256
+#define LOOP_CARRY_CTAS 32   // CTAs per sequence of the pyramid carry of a listed step
 
 struct LoopOut {   // per-sequence results of a step: the packed block of b200vo_loop_step or the caller's device arrays
     int* status; int* n_inl; int* n_lm; int* n_cand; double* pose;
@@ -46,15 +48,45 @@ struct LoopDev {   // kernel view of the state and of the step's scratch (device
     uint8_t* keep; float* new_lm; float* new_kp; int* n_new;                      // its outputs ([batch][C]...)
     const float* corners; const int* gftt_small;                                  // detector output
     int* n_corner; uint8_t* valid;             // corners per sequence, distance-filter result [batch][G]
+    // a listed step: its sequences (one CTA each, result row = CTA), nullptr: every sequence; the tracker counts of the
+    // step (trk_lm / trk_cand of the listed sequences, 0 for the others)
+    const int* list;
+    int* step_lm; int* step_cand;
 };
+
+// The sequence of CTA `blockIdx.x` of a loop kernel: the listed sequence of that row, or the CTA's own index
+__device__ __forceinline__ int loop_seq(const LoopDev& d) { return d.list ? d.list[blockIdx.x] : (int)blockIdx.x; }
+
+// The first kernel of a listed step.  Every sequence: the tracker counts of the step (its trk_lm / trk_cand when listed, 0
+// otherwise: the trackers and the pose chain do no work for it), and for one that is not listed no triangulation and no
+// distance filter (tri_n and n_corner still hold its last listed step's values).  Every sequence that is not listed also
+// gets its current pyramid carried from the previous frames' slab set into this step's, so that after the step set `cur`
+// holds every sequence's current pyramid again.  Grid (x, batch); pos = the list row's [batch] positions.
+__global__ void __launch_bounds__(256)
+loop_list_kernel(LoopDev d, const int* __restrict__ pos, const uint4* __restrict__ cur_slab, uint4* __restrict__ nxt_slab,
+                 size_t slab_words)
+{
+    const int s = blockIdx.y;
+    const bool listed = pos[s] >= 0;
+    if (blockIdx.x == 0 && threadIdx.x == 0) {
+        d.step_lm[s] = listed ? d.trk_lm[s] : 0;
+        d.step_cand[s] = listed ? d.trk_cand[s] : 0;
+        if (!listed) { d.tri_n[s] = 0; d.n_corner[s] = 0; }
+    }
+    if (listed) return;
+    const uint4* src = cur_slab + (size_t)s * slab_words;
+    uint4* dst = nxt_slab + (size_t)s * slab_words;
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < slab_words; i += (size_t)gridDim.x * blockDim.x) dst[i] = src[i];
+}
 
 // Steps 3-5 of MiniVO.step and the status filter of step 2: one CTA per sequence.
 __global__ void __launch_bounds__(LOOP_T)
 loop_commit_kernel(LoopDev d, LoopOut out)
 {
-    __shared__ int s_code;
-    const int s = blockIdx.x, tid = threadIdx.x;
+    __shared__ int s_code, s_seq;
+    const int s = loop_seq(d), r = blockIdx.x, tid = threadIdx.x;
     if (tid == 0) {
+        s_seq = s;
         int code = d.status[s];
         if (code == B200VO_LOOP_OK) {
             if (d.c_n[s] < 8) code = B200VO_LOOP_FEW_POINTS;
@@ -72,12 +104,13 @@ loop_commit_kernel(LoopDev d, LoopOut out)
         const double* rt = d.pose6 + 6 * s;
         double R[9], cw[12];
         vo::rodrigues_to_R(rt, R);
+        const int s = *(volatile int*)&s_seq;   // read again: a listed sequence index kept live across the call would spill
         for (int i = 0; i < 3; ++i)
             for (int j = 0; j < 3; ++j) cw[3 * i + j] = R[3 * j + i];
         for (int i = 0; i < 3; ++i) cw[9 + i] = -R[i] * rt[3] + -R[3 + i] * rt[4] + -R[6 + i] * rt[5];
         double* hist = d.poses + ((size_t)s * d.P + d.n_poses[s]) * 12;   // appended by loop_append_kernel
-        for (int k = 0; k < 12; ++k) { d.cur_pose[12 * s + k] = cw[k]; hist[k] = cw[k]; out.pose[12 * s + k] = cw[k]; }
-        out.n_inl[s] = d.n_inl[s];
+        for (int k = 0; k < 12; ++k) { d.cur_pose[12 * s + k] = cw[k]; hist[k] = cw[k]; out.pose[12 * r + k] = cw[k]; }
+        out.n_inl[r] = d.n_inl[s];
         d.n_corner[s] = d.gftt_small[s * VO_GFTT_SMALL + 2];
     }
     // the inliers of the tracked landmarks, in order (:346-350)
@@ -109,7 +142,7 @@ loop_commit_kernel(LoopDev d, LoopOut out)
 __global__ void __launch_bounds__(LOOP_T)
 loop_merge_kernel(LoopDev d)
 {
-    const int s = blockIdx.x, tid = threadIdx.x;
+    const int s = loop_seq(d), tid = threadIdx.x;
     if (d.status[s] != B200VO_LOOP_OK) return;   // written by this kernel only by thread 0, after every read below
     const bool ran = d.tri_n[s] > 0;
     const int nn = ran ? d.n_new[s] : 0, nl = d.n_lm[s];
@@ -140,7 +173,7 @@ __global__ void __launch_bounds__(LOOP_T)
 loop_append_kernel(LoopDev d, LoopOut out)
 {
     __shared__ int s_st;
-    const int s = blockIdx.x, tid = threadIdx.x;
+    const int s = loop_seq(d), r = blockIdx.x, tid = threadIdx.x;
     if (tid == 0) s_st = d.status[s];
     __syncthreads();
     if (s_st == B200VO_LOOP_OK) {
@@ -162,10 +195,10 @@ loop_append_kernel(LoopDev d, LoopOut out)
     }
     if (tid == 0) {
         const int st = s_st, nl = d.n_lm[s], nc = d.n_cand[s];
-        out.status[s] = st; out.n_lm[s] = nl; out.n_cand[s] = nc;
+        out.status[r] = st; out.n_lm[r] = nl; out.n_cand[r] = nc;
         if (st != B200VO_LOOP_OK) {
-            out.n_inl[s] = 0;
-            for (int k = 0; k < 12; ++k) out.pose[12 * s + k] = 0.0;
+            out.n_inl[r] = 0;
+            for (int k = 0; k < 12; ++k) out.pose[12 * r + k] = 0.0;
         }
         d.trk_lm[s] = st == B200VO_LOOP_OK ? nl : 0;
         d.trk_cand[s] = st == B200VO_LOOP_OK && nc > 1 ? nc : 0;   // the reference tracks candidates only when n > 1 (:286)
@@ -176,7 +209,7 @@ loop_append_kernel(LoopDev d, LoopOut out)
 // host side
 // ------------------------------------------------------------------------------------------
 enum { CNT_LM, CNT_CAND, CNT_POSES, CNT_STATUS, CNT_TRK_LM, CNT_TRK_CAND, CNT_INL, CNT_CAND_B, CNT_TRI, CNT_NEW, CNT_CORNER,
-       CNT_FLAGS, CNT_KINDS };
+       CNT_FLAGS, CNT_STEP_LM, CNT_STEP_CAND, CNT_KINDS };
 
 struct b200vo_loop {
     b200vo_ctx* ctx = nullptr;
@@ -229,6 +262,7 @@ extern "C" int b200vo_loop_create(b200vo_ctx* ctx, int batch, const b200vo_loop_
     lp->res_bytes = nb * 96 + 4 * nb * 4;
     if (!rc) rc = vo_reserve(ctx, lp->res, lp->res_bytes);
     if (!rc) rc = vo_reserve(ctx, B->gftt_ws, vo_gftt_batch_workspace(bc.rows, bc.cols, batch, cfg->max_corners));
+    if (!rc) rc = vo_reserve(ctx, B->lists, 3 * 2 * nb * sizeof(int32_t));
     if (rc) { b200vo_loop_destroy(lp); return rc; }
     uint8_t* p = (uint8_t*)lp->mem.p;
     int k = 0;
@@ -244,6 +278,7 @@ extern "C" int b200vo_loop_create(b200vo_ctx* ctx, int batch, const b200vo_loop_
     d.n_lm = cnt + CNT_LM * nb; d.n_cand = cnt + CNT_CAND * nb; d.n_poses = cnt + CNT_POSES * nb; d.status = cnt + CNT_STATUS * nb;
     d.trk_lm = cnt + CNT_TRK_LM * nb; d.trk_cand = cnt + CNT_TRK_CAND * nb; d.n_inl = cnt + CNT_INL * nb;
     d.n_cand_b = cnt + CNT_CAND_B * nb; d.tri_n = cnt + CNT_TRI * nb; d.n_new = cnt + CNT_NEW * nb; d.n_corner = cnt + CNT_CORNER * nb;
+    d.step_lm = cnt + CNT_STEP_LM * nb; d.step_cand = cnt + CNT_STEP_CAND * nb;
     d.c_obj = B->c_obj; d.c_img = B->c_img; d.c_n = B->c_n; d.inliers = B->inliers;
     TriBatchArgs& t = lp->tri;
     vo_tri_common(t.common, cfg->min_dist_landmarks, cfg->max_dist_landmarks, cfg->min_baseline_angle_deg, cfg->min_baseline_frames);
@@ -270,41 +305,63 @@ extern "C" int b200vo_loop_create(b200vo_ctx* ctx, int batch, const b200vo_loop_
     return 0;
 }
 
-// one step of every sequence, enqueued on the ctx stream (the tracker and the pose chain use the batch object's streams
-// and join it); frames_dev == nullptr: the oldest submitted frame set
-static int loop_core(b200vo_loop* lp, const uint8_t* frames_dev, const LoopOut& o)
+// one step of every sequence, or with n_list > 0 of the sequences list[0 .. n_list) (validated), enqueued on the ctx stream
+// (the tracker and the pose chain use the batch object's streams and join it); frames_dev == nullptr: the oldest submitted
+// frame set.  Result row k belongs to the k-th sequence of the step.
+static int loop_core(b200vo_loop* lp, const uint8_t* frames_dev, const LoopOut& o, int n_list = 0, const int32_t* list = nullptr)
 {
     b200vo_ctx* ctx = lp->ctx;
     b200vo_batch* B = lp->B;
     const b200vo_loop_cfg& c = lp->cfg;
     LoopDev& d = lp->d;
     const int nb = lp->batch;
-    VO_TRY(batch_select_frames(B, frames_dev));
-    VO_TRY(batch_track_pose_overlapped(B, frames_dev, d.lm_kp, d.lm, d.trk_lm, d.keys, d.trk_cand, d.lm_next, d.lm_status, d.cand_next,
+    VO_TRY(batch_select_frames(B, frames_dev, n_list, list));
+    d.list = B->step_list;
+    const int n_cta = d.list ? B->step_n : nb;
+    if (d.list) {
+        const size_t words = B->geom.slab_bytes / 16;
+        loop_list_kernel<<<dim3(LOOP_CARRY_CTAS, nb), 256, 0, ctx->stream>>>(d, d.list + nb, (const uint4*)B->slabs[B->cur].p,
+                                                                             (uint4*)B->slabs[B->nxt].p, words);
+        ctx->launches++;
+    }
+    const int* trk_lm = d.list ? d.step_lm : d.trk_lm;
+    const int* trk_cand = d.list ? d.step_cand : d.trk_cand;
+    VO_TRY(batch_track_pose_overlapped(B, frames_dev, d.lm_kp, d.lm, trk_lm, d.keys, trk_cand, d.lm_next, d.lm_status, d.cand_next,
                                        d.cand_status, d.pose6, d.pnp_ok, d.inl_mask, d.n_inl, nullptr));
     float* corners = nullptr;
     int* small = nullptr;
     VO_TRY(vo_gftt_batch_launch(ctx, (const uint8_t*)B->slabs[B->nxt].p + B->geom.off[0], B->geom.slab_bytes, B->geom.pitch[0],
                                 c.batch.rows, c.batch.cols, nb, c.max_corners, c.quality_level, c.feature_min_dist, B->gftt_ws.p,
-                                &corners, &small, B->ext));
+                                &corners, &small, B->ext, d.list, n_cta));
     d.corners = corners; d.gftt_small = small;
-    loop_commit_kernel<<<nb, LOOP_T, 0, ctx->stream>>>(d, o);
+    loop_commit_kernel<<<n_cta, LOOP_T, 0, ctx->stream>>>(d, o);
     ctx->launches++;
     VO_TRY(vo_triangulate_batch_launch(ctx, lp->tri, nb, ctx->stream));
-    loop_merge_kernel<<<nb, LOOP_T, 0, ctx->stream>>>(d);
+    loop_merge_kernel<<<n_cta, LOOP_T, 0, ctx->stream>>>(d);
     ctx->launches++;
     VO_TRY(vo_min_distance_batch_launch(ctx, nb, d.corners, d.n_corner, d.G, d.keys, d.n_cand, d.C, (float)c.feature_min_dist, d.valid,
                                         ctx->stream));
-    loop_append_kernel<<<nb, LOOP_T, 0, ctx->stream>>>(d, o);
+    loop_append_kernel<<<n_cta, LOOP_T, 0, ctx->stream>>>(d, o);
     ctx->launches++;
     VO_CUDA(ctx, cudaGetLastError());
     return batch_finish(B);
+}
+
+// a full step must not consume a set that was submitted with a list
+static int loop_check_full(b200vo_loop* lp, const uint8_t* frames)
+{
+    const b200vo_batch* B = lp->B;
+    if (!frames && B->q_count > 0 && !B->q_list[B->q_head].empty())
+        return vo_set_err(lp->ctx, B200VO_E_BADARG, "the oldest submitted frame set lists %d sequences: consume it with the listed step",
+                          (int)B->q_list[B->q_head].size());
+    return 0;
 }
 
 extern "C" int b200vo_loop_step_dev(b200vo_loop* lp, const uint8_t* frames_dev, int32_t* status_dev, int32_t* n_inliers_dev,
                                     int32_t* n_lm_dev, int32_t* n_cand_dev, double* pose_cw_dev)
 {
     if (!lp || !status_dev || !n_inliers_dev || !n_lm_dev || !n_cand_dev || !pose_cw_dev) return B200VO_E_BADARG;
+    VO_TRY(loop_check_full(lp, frames_dev));
     VO_CUDA(lp->ctx, cudaSetDevice(lp->ctx->device));
     const LoopOut o{status_dev, n_inliers_dev, n_lm_dev, n_cand_dev, pose_cw_dev};
     return loop_core(lp, frames_dev, o);
@@ -314,6 +371,7 @@ extern "C" int b200vo_loop_step(b200vo_loop* lp, const uint8_t* frames, int32_t*
                                 int32_t* n_cand, double* pose_cw)
 {
     if (!lp || !status || !n_inliers || !n_lm || !n_cand || !pose_cw) return B200VO_E_BADARG;
+    VO_TRY(loop_check_full(lp, frames));
     b200vo_ctx* ctx = lp->ctx;
     b200vo_batch* B = lp->B;
     VO_CUDA(ctx, cudaSetDevice(ctx->device));
@@ -360,6 +418,114 @@ extern "C" int b200vo_loop_submit_frames(b200vo_loop* lp, const uint8_t* frames)
 extern "C" int b200vo_loop_submit_frames_dev(b200vo_loop* lp, const uint8_t* frames_dev)
 {
     return lp ? batch_submit(lp->B, frames_dev, true) : B200VO_E_BADARG;
+}
+
+// ------------------------------------------------------------------------------------------
+// listed steps: only the sequences of a list advance
+// ------------------------------------------------------------------------------------------
+// n_seq distinct indices in [0, batch)
+static int loop_check_list(b200vo_loop* lp, int n_seq, const int32_t* seqs)
+{
+    b200vo_ctx* ctx = lp->ctx;
+    if (n_seq < 1 || n_seq > lp->batch) return vo_set_err(ctx, B200VO_E_BADARG, "n_seq = %d is outside [1, batch = %d]", n_seq, lp->batch);
+    if (!seqs) return vo_set_err(ctx, B200VO_E_BADARG, "null array");
+    std::vector<char> seen(lp->batch, 0);
+    for (int k = 0; k < n_seq; ++k) {
+        if (seqs[k] < 0 || seqs[k] >= lp->batch)
+            return vo_set_err(ctx, B200VO_E_BADARG, "seqs[%d] = %d is outside [0, batch = %d)", k, seqs[k], lp->batch);
+        if (seen[seqs[k]]++) return vo_set_err(ctx, B200VO_E_BADARG, "sequence %d is listed twice", seqs[k]);
+    }
+    return 0;
+}
+
+// what a listed step may consume: its own frames while no set waits, or the oldest submitted set if it has the same list
+static int loop_check_step_list(b200vo_loop* lp, int n_seq, const int32_t* seqs, const uint8_t* frames)
+{
+    b200vo_ctx* ctx = lp->ctx;
+    const b200vo_batch* B = lp->B;
+    VO_TRY(loop_check_list(lp, n_seq, seqs));
+    if (frames) {
+        if (B->q_count > 0)
+            return vo_set_err(ctx, B200VO_E_BADARG, "submitted frame sets are waiting: pass frames == NULL to consume them in order");
+        return 0;
+    }
+    if (B->q_count == 0) return vo_set_err(ctx, B200VO_E_BADARG, "frames == NULL but no frame set was submitted");
+    const std::vector<int32_t>& q = B->q_list[B->q_head];
+    if (q.empty()) return vo_set_err(ctx, B200VO_E_BADARG, "the oldest submitted frame set covers every sequence: consume it with the full step");
+    if ((int)q.size() != n_seq || !std::equal(q.begin(), q.end(), seqs))
+        return vo_set_err(ctx, B200VO_E_BADARG, "the oldest submitted frame set was submitted with another list");
+    return 0;
+}
+
+extern "C" int b200vo_loop_step_seqs_dev(b200vo_loop* lp, int n_seq, const int32_t* seqs, const uint8_t* frames_dev, int32_t* status_dev,
+                                         int32_t* n_inliers_dev, int32_t* n_lm_dev, int32_t* n_cand_dev, double* pose_cw_dev)
+{
+    if (!lp) return B200VO_E_BADARG;
+    if (!status_dev || !n_inliers_dev || !n_lm_dev || !n_cand_dev || !pose_cw_dev) return vo_set_err(lp->ctx, B200VO_E_BADARG, "null array");
+    VO_TRY(loop_check_step_list(lp, n_seq, seqs, frames_dev));
+    VO_CUDA(lp->ctx, cudaSetDevice(lp->ctx->device));
+    const LoopOut o{status_dev, n_inliers_dev, n_lm_dev, n_cand_dev, pose_cw_dev};
+    return loop_core(lp, frames_dev, o, n_seq, seqs);
+}
+
+extern "C" int b200vo_loop_step_seqs(b200vo_loop* lp, int n_seq, const int32_t* seqs, const uint8_t* frames, int32_t* status,
+                                     int32_t* n_inliers, int32_t* n_lm, int32_t* n_cand, double* pose_cw)
+{
+    if (!lp) return B200VO_E_BADARG;
+    b200vo_ctx* ctx = lp->ctx;
+    b200vo_batch* B = lp->B;
+    if (!status || !n_inliers || !n_lm || !n_cand || !pose_cw) return vo_set_err(ctx, B200VO_E_BADARG, "null array");
+    VO_TRY(loop_check_step_list(lp, n_seq, seqs, frames));
+    VO_CUDA(ctx, cudaSetDevice(ctx->device));
+    VO_CUDA(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
+    const size_t ns = n_seq, f_total = (size_t)lp->cfg.batch.rows * lp->cfg.batch.cols * ns;
+    bool pinned = false;
+    if (frames) {
+        cudaPointerAttributes at{};
+        pinned = cudaPointerGetAttributes(&at, frames) == cudaSuccess && at.type == cudaMemoryTypeHost;
+        cudaGetLastError();
+    }
+    // the result rows of the listed sequences, packed as the full step's block: pose_cw [n_seq][12] | status | n_inliers | n_lm | n_cand
+    uint8_t* r = (uint8_t*)lp->res.p;
+    const LoopOut o{(int*)(r + ns * 96), (int*)(r + ns * 96) + ns, (int*)(r + ns * 96) + 2 * ns, (int*)(r + ns * 96) + 3 * ns, (double*)r};
+    const size_t res_bytes = ns * 96 + 4 * ns * 4;
+    const size_t staged = frames && !pinned ? vo_align(f_total, 256) : 0;
+    VO_TRY(vo_reserve_pinned(ctx, staged + res_bytes));
+    uint8_t* hp = (uint8_t*)ctx->h_pin;
+    const uint8_t* fdev = nullptr;
+    if (frames) {   // the one upload of the step: the listed frames
+        VO_TRY(vo_reserve(ctx, B->raw, f_total));
+        if (!pinned) memcpy(hp, frames, f_total);
+        VO_CUDA(ctx, cudaMemcpyAsync(B->raw.p, pinned ? frames : hp, f_total, cudaMemcpyHostToDevice, ctx->stream));
+        fdev = (const uint8_t*)B->raw.p;
+    }
+    VO_TRY(loop_core(lp, fdev, o, n_seq, seqs));
+    uint8_t* ho = hp + staged;   // the one read-back of the step
+    VO_CUDA(ctx, cudaMemcpyAsync(ho, r, res_bytes, cudaMemcpyDeviceToHost, ctx->stream));
+    VO_CUDA(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
+    VO_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    cudaEventElapsedTime(&ctx->last_ms, ctx->ev0, ctx->ev1);
+    memcpy(pose_cw, ho, ns * 96);
+    const int* ri = (const int*)(ho + ns * 96);
+    memcpy(status, ri, ns * 4);
+    memcpy(n_inliers, ri + ns, ns * 4);
+    memcpy(n_lm, ri + 2 * ns, ns * 4);
+    memcpy(n_cand, ri + 3 * ns, ns * 4);
+    return 0;
+}
+
+extern "C" int b200vo_loop_submit_frames_seqs(b200vo_loop* lp, int n_seq, const int32_t* seqs, const uint8_t* frames)
+{
+    if (!lp) return B200VO_E_BADARG;
+    VO_TRY(loop_check_list(lp, n_seq, seqs));
+    return batch_submit(lp->B, frames, false, n_seq, seqs);
+}
+
+extern "C" int b200vo_loop_submit_frames_seqs_dev(b200vo_loop* lp, int n_seq, const int32_t* seqs, const uint8_t* frames_dev)
+{
+    if (!lp) return B200VO_E_BADARG;
+    VO_TRY(loop_check_list(lp, n_seq, seqs));
+    return batch_submit(lp->B, frames_dev, true, n_seq, seqs);
 }
 
 extern "C" int b200vo_loop_load(b200vo_loop* lp, int seq, const uint8_t* frame, const float* lm, const float* lm_kp, int n_lm,

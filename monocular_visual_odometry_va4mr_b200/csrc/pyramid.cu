@@ -70,14 +70,15 @@ __device__ __forceinline__ int reflect101(int p, int len)
 }
 
 // raw image (rows of raw_row bytes) -> bordered level 0.  One thread = one 16-byte store of the bordered row.
-// ext: the sequence's own width and height (the grid covers the slot's)
+// ext: the sequence's own width and height (the grid covers the slot's); list: raw image z goes to slab list[z]
 __global__ void __launch_bounds__(256)
 pad_level0_kernel(const uint8_t* __restrict__ raw, size_t raw_stride, size_t raw_row, int w, int h,
-                  uint8_t* __restrict__ slab, size_t slab_stride, size_t off0, int pitch, const VoSeqExt* __restrict__ ext)
+                  uint8_t* __restrict__ slab, size_t slab_stride, size_t off0, int pitch, const VoSeqExt* __restrict__ ext,
+                  const int* __restrict__ list)
 {
-    const int seq = blockIdx.z;
+    const int seq = list ? list[blockIdx.z] : blockIdx.z;
     if (ext) { w = ext[seq].w[0]; h = ext[seq].h[0]; }
-    const uint8_t* src = raw + seq * raw_stride;
+    const uint8_t* src = raw + blockIdx.z * raw_stride;
     uint8_t* dst = slab + seq * slab_stride + off0;
     const int gx = (blockIdx.x * blockDim.x + threadIdx.x) * 16 - VO_BORDER;  // first of 16 px
     const int gy = blockIdx.y * blockDim.y + threadIdx.y - VO_BORDER;
@@ -114,9 +115,9 @@ pad_level0_kernel(const uint8_t* __restrict__ raw, size_t raw_stride, size_t raw
 __global__ void __launch_bounds__(256)
 pyr_down_kernel(const uint8_t* __restrict__ slab_src, uint8_t* __restrict__ slab_dst, size_t slab_stride,
                 size_t off_s, int sw, int sh, int spitch, size_t off_d, int dw, int dh, int dpitch,
-                const VoSeqExt* __restrict__ ext, int level)
+                const VoSeqExt* __restrict__ ext, int level, const int* __restrict__ list)
 {
-    const int seq = blockIdx.z;
+    const int seq = list ? list[blockIdx.z] : blockIdx.z;
     if (ext) {   // the sequence's own level `level` from its level - 1; nothing beyond its level count
         if (level >= ext[seq].levels) return;
         dw = ext[seq].w[level]; dh = ext[seq].h[level];
@@ -178,12 +179,13 @@ pyr_down_kernel(const uint8_t* __restrict__ slab_src, uint8_t* __restrict__ slab
 
 __global__ void __launch_bounds__(256)
 pyr_down_tma_kernel(const __grid_constant__ CUtensorMap src_map, uint8_t* __restrict__ slab_dst, size_t slab_stride,
-                    size_t off_d, int dw, int dh, int dpitch, int fuse_border, const VoSeqExt* __restrict__ ext, int level)
+                    size_t off_d, int dw, int dh, int dpitch, int fuse_border, const VoSeqExt* __restrict__ ext, int level,
+                    const int* __restrict__ list)
 {
     // source bytes [0,160) and [128,288) of each row; each half starts on a 128-byte boundary (TMA destination)
     __shared__ __align__(128) uint8_t tile[2][(PD_SR * PD_SB + 127) / 128 * 128];
     __shared__ __align__(8) unsigned long long bar;
-    const int seq = blockIdx.z;
+    const int seq = list ? list[blockIdx.z] : blockIdx.z;   // the slab, and the map's third coordinate
     const int X0 = blockIdx.x * PD_TW, Y0 = blockIdx.y * PD_TH;
     if (ext) {   // the sequence's own extents of this level: tiles outside them (and levels beyond its count) exit
         if (level >= ext[seq].levels) return;
@@ -263,17 +265,19 @@ pyr_down_tma_kernel(const __grid_constant__ CUtensorMap src_map, uint8_t* __rest
 // tracker's window reads depend on it)
 struct BorderArgs { int levels; int w[VO_MAX_LEVELS], h[VO_MAX_LEVELS], pitch[VO_MAX_LEVELS]; unsigned long long off[VO_MAX_LEVELS]; };
 __global__ void __launch_bounds__(256)
-pyr_border_level_kernel(uint8_t* __restrict__ slab, size_t slab_stride, BorderArgs a, int level, const VoSeqExt* __restrict__ ext)
+pyr_border_level_kernel(uint8_t* __restrict__ slab, size_t slab_stride, BorderArgs a, int level, const VoSeqExt* __restrict__ ext,
+                        const int* __restrict__ list)
 {
     int w = a.w[level], h = a.h[level];
     const int pitch = a.pitch[level];
+    const int seq = list ? list[blockIdx.z] : blockIdx.z;
     if (ext) {   // only the sequences whose level was not given its ring by the tiles
-        const VoSeqExt& e = ext[blockIdx.z];
+        const VoSeqExt& e = ext[seq];
         if (level >= e.levels) return;
         w = e.w[level]; h = e.h[level];
         if (w >= VO_BORDER + 2 && h >= VO_BORDER + 2) return;
     }
-    uint8_t* base = slab + blockIdx.z * slab_stride + a.off[level];
+    uint8_t* base = slab + seq * slab_stride + a.off[level];
     // ring in aligned 4-byte words: top + bottom bands over the full bordered width, then per interior
     // row 8 words on the left (x = -32..-1) and 9 on the right (from x = w & ~3, covering w .. w+31)
     const int wq = (w + 2 * VO_BORDER + 3) / 4;
@@ -323,33 +327,37 @@ static int pyr_src_map(b200vo_ctx* ctx, CUtensorMap* map, uint8_t* d_slab, size_
 
 int vo_build_pyramids(b200vo_ctx* ctx, const uint8_t* d_raw, size_t raw_stride, int rows, int cols,
                       const PyrGeom& g, uint8_t* d_slab, size_t slab_stride, int batch, cudaStream_t stream,
-                      const VoSeqExt* d_ext, const VoSeqExt* h_ext, size_t raw_row)
+                      const VoSeqExt* d_ext, const VoSeqExt* h_ext, size_t raw_row, const int* d_list, const int* h_list, int n_slab)
 {
     if (!raw_row) raw_row = (size_t)cols;
+    // the slabs the tensor maps span: every slab of the set when the images go to listed slabs
+    const int n_map = d_list ? n_slab : batch;
     {
         dim3 block(32, 8);
         int gxn = (cols + 2 * VO_BORDER + 15) / 16;
         dim3 grid((gxn + block.x - 1) / block.x, (rows + 2 * VO_BORDER + block.y - 1) / block.y, batch);
         pad_level0_kernel<<<grid, block, 0, stream>>>(d_raw, raw_stride, raw_row, cols, rows, d_slab, slab_stride,
-                                                       g.off[0], g.pitch[0], d_ext);
+                                                       g.off[0], g.pitch[0], d_ext, d_list);
         ctx->launches++;
     }
     if (g.levels > 1) {
         // TMA needs 16-byte aligned strides and base: slab strides are multiples of 256, pitches of 128
-        const bool tma_ok = (slab_stride % 16 == 0 || batch == 1) && (reinterpret_cast<uintptr_t>(d_slab) % 256 == 0);
+        const bool tma_ok = (slab_stride % 16 == 0 || n_map == 1) && (reinterpret_cast<uintptr_t>(d_slab) % 256 == 0);
         for (int l = 1; l < g.levels; ++l) {
             bool fused = false;
             if (tma_ok) {
                 CUtensorMap map;
-                VO_TRY(pyr_src_map(ctx, &map, d_slab, batch == 1 ? g.slab_bytes : slab_stride, batch, g, l - 1));
+                VO_TRY(pyr_src_map(ctx, &map, d_slab, n_map == 1 ? g.slab_bytes : slab_stride, n_map, g, l - 1));
                 dim3 grid((g.w[l] + PD_TW - 1) / PD_TW, (g.h[l] + PD_TH - 1) / PD_TH, batch);
                 fused = g.w[l] >= VO_BORDER + 2 && g.h[l] >= VO_BORDER + 2;   // single-bounce reflection: the tiles write the ring
                 pyr_down_tma_kernel<<<grid, 256, 0, stream>>>(map, d_slab, slab_stride, g.off[l], g.w[l], g.h[l], g.pitch[l], fused ? 1 : 0,
-                                                              d_ext, l);
+                                                              d_ext, l, d_list);
                 if (h_ext) {   // the single-bounce test per sequence: a ring is left to the border kernel if any tile set could not write it
                     fused = true;
-                    for (int b = 0; b < batch; ++b)
-                        if (l < h_ext[b].levels && !(h_ext[b].w[l] >= VO_BORDER + 2 && h_ext[b].h[l] >= VO_BORDER + 2)) fused = false;
+                    for (int b = 0; b < batch; ++b) {
+                        const VoSeqExt& e = h_ext[h_list ? h_list[b] : b];
+                        if (l < e.levels && !(e.w[l] >= VO_BORDER + 2 && e.h[l] >= VO_BORDER + 2)) fused = false;
+                    }
                 }
             } else {
                 dim3 block(32, 8);
@@ -357,7 +365,7 @@ int vo_build_pyramids(b200vo_ctx* ctx, const uint8_t* d_raw, size_t raw_stride, 
                 dim3 grid((gxn + block.x - 1) / block.x, (g.h[l] + 2 * VO_BORDER + block.y - 1) / block.y, batch);
                 pyr_down_kernel<<<grid, block, 0, stream>>>(d_slab, d_slab, slab_stride, g.off[l - 1], g.w[l - 1],
                                                              g.h[l - 1], g.pitch[l - 1], g.off[l], g.w[l], g.h[l],
-                                                             g.pitch[l], d_ext, l);
+                                                             g.pitch[l], d_ext, l, d_list);
             }
             ctx->launches++;
             if (tma_ok && !fused) {
@@ -367,7 +375,7 @@ int vo_build_pyramids(b200vo_ctx* ctx, const uint8_t* d_raw, size_t raw_stride, 
                 for (int k = 0; k <= l; ++k) { ba.w[k] = g.w[k]; ba.h[k] = g.h[k]; ba.pitch[k] = g.pitch[k]; ba.off[k] = g.off[k]; }
                 // only level l needs filling now: launch with a single y-slice mapped onto level l
                 ba.levels = l + 1;
-                pyr_border_level_kernel<<<dim3(16, 1, batch), 256, 0, stream>>>(d_slab, slab_stride, ba, l, d_ext);
+                pyr_border_level_kernel<<<dim3(16, 1, batch), 256, 0, stream>>>(d_slab, slab_stride, ba, l, d_ext, d_list);
                 ctx->launches++;
             }
         }
