@@ -78,6 +78,17 @@ int b200vo_frame_download_level(b200vo_ctx* ctx, int slot, int level, uint8_t* o
 int b200vo_good_features_to_track(b200vo_ctx* ctx, const uint8_t* img, int rows, int cols,
                                   size_t step, int max_corners, double quality, double min_dist,
                                   int block_size, float* corners_xy, int* n_out);
+/*
+ * The same with cv2's detection mask (goodFeaturesToTrack(..., mask=)): mask uint8 (rows, cols), `mask_step` bytes a row.
+ * A corner needs a nonzero mask byte at its pixel (any nonzero value counts), and the quality threshold is qualityLevel
+ * times the largest eigenvalue over the pixels of nonzero bytes only (1-pixel border included), as cv2's
+ * minMaxLoc(eig, mask): a masked-out region does not set it.  An all-zero mask gives no corners.  mask == NULL behaves
+ * as b200vo_good_features_to_track.  The mask must have the image's size (the caller checks it; cv2 raises otherwise).
+ */
+int b200vo_good_features_to_track_masked(b200vo_ctx* ctx, const uint8_t* img, int rows, int cols,
+                                         size_t step, const uint8_t* mask, size_t mask_step,
+                                         int max_corners, double quality, double min_dist,
+                                         int block_size, float* corners_xy, int* n_out);
 
 /*
  * Replaces cv2.BFMatcher().knnMatch(desc0, desc1, k=2) at :229 plus the Lowe ratio loop at
@@ -212,6 +223,15 @@ int b200vo_recover_pose(b200vo_ctx* ctx, const double E[9], const float* p1, con
  */
 int b200vo_sift_detect_and_compute(b200vo_ctx* ctx, const uint8_t* img, int rows, int cols, size_t step, int max_kp,
                                    float* kps, float* desc, int32_t* n_out);
+/*
+ * The same with cv2's detection mask (detectAndCompute(img, mask)): mask uint8 (rows, cols), `mask_step` bytes a row.  As
+ * cv2's KeyPointsFilter::runByPixelsMask after the duplicate removal, a keypoint is dropped when the mask byte at
+ * ((int)(y + 0.5f), (int)(x + 0.5f)) is 0; the others keep their order and descriptors, and *n_out counts them.
+ * mask == NULL behaves as b200vo_sift_detect_and_compute.  The mask must have the image's size (cv2 does not check it).
+ */
+int b200vo_sift_detect_and_compute_masked(b200vo_ctx* ctx, const uint8_t* img, int rows, int cols, size_t step,
+                                          const uint8_t* mask, size_t mask_step, int max_kp, float* kps,
+                                          float* desc, int32_t* n_out);
 
 /*
  * Replaces cv2.solvePnPRansac(obj, img, K, zeros(4), flags=SOLVEPNP_P3P, confidence=,
@@ -270,9 +290,23 @@ int b200vo_batch_set_intrinsics(b200vo_batch* b, int n_seq, const int32_t* seqs,
  * read, and it is tracked and detected exactly as in a batch of its own size (its own pyramid level count included).
  * A size must fit the slot and be larger than the window (cfg->win_h x cfg->win_w).  Bad indices (out of range, repeated),
  * n_seq < 1, null arrays, a bad size or submitted frame sets still waiting: B200VO_E_BADARG and nothing changes.
- * The resident frames no longer match: the next step needs b200vo_batch_prime.  Synchronous.
+ * The resident frames no longer match: the next step needs b200vo_batch_prime.  The listed sequences' detection masks
+ * are cleared (a mask has its sequence's frame size).  Synchronous.
  */
 int b200vo_batch_set_frame_size(b200vo_batch* b, int n_seq, const int32_t* seqs, const int32_t* rows, const int32_t* cols);
+/*
+ * Per-sequence detection mask (cv2's goodFeaturesToTrack(..., mask=)), for static regions whose corners move with the
+ * camera: a car's hood, the black wedges of an undistorted image, a burned-in timestamp or logo.  masks: uint8
+ * [n_seq][cfg->rows][cfg->cols] in the slot layout; sequence seqs[k]'s mask is the top-left of row k at its own frame size
+ * (bytes outside it are never read).  b200vo_batch_good_features then detects in that sequence exactly as
+ * b200vo_good_features_to_track_masked on its frame and mask.  masks == NULL clears the listed sequences' masks.  The mask
+ * gates detection only: tracking and pose do not read it.  Bad indices (out of range, repeated), n_seq < 1 or a null seqs:
+ * B200VO_E_BADARG and nothing changes.  The mask memory (batch x rows x cols bytes) is allocated with the first mask; a
+ * batch without masks runs the detector without mask reads.  Synchronous (waits for the step in flight).  Unlike a frame
+ * size, a mask may change while submitted frame sets wait: it applies to every step that runs after the call, those sets'
+ * steps included, as the frames' pyramids do not depend on it.
+ */
+int b200vo_batch_set_detection_mask(b200vo_batch* b, int n_seq, const int32_t* seqs, const uint8_t* masks);
 /* Upload the first frame of every sequence (frames: batch x rows x cols, tight). */
 int b200vo_batch_prime(b200vo_batch* b, const uint8_t* frames);
 /*
@@ -364,8 +398,13 @@ void b200vo_loop_destroy(b200vo_loop* lp);
 int b200vo_loop_set_intrinsics(b200vo_loop* lp, int n_seq, const int32_t* seqs, const double* K);
 /* Per-sequence frame size of the loop, as b200vo_batch_set_frame_size (same validation: B200VO_E_BADARG, nothing changes).
  * The listed sequences become B200VO_LOOP_IDLE: their state arrays stay readable, and steps skip them until
- * b200vo_loop_load or b200vo_loop_bootstrap runs for them.  Synchronous. */
+ * b200vo_loop_load or b200vo_loop_bootstrap runs for them.  Their detection masks are cleared.  Synchronous. */
 int b200vo_loop_set_frame_size(b200vo_loop* lp, int n_seq, const int32_t* seqs, const int32_t* rows, const int32_t* cols);
+/* Per-sequence detection mask of the loop, as b200vo_batch_set_detection_mask (same layout and validation).  It applies to
+ * the corners a step detects for feature adding and to both SIFT frames of b200vo_loop_bootstrap, so that a sequence's
+ * results are those of the per-call masked forms on its frames; tracking, pose and triangulation do not read it.  The
+ * state, status and frames are not touched.  Synchronous. */
+int b200vo_loop_set_detection_mask(b200vo_loop* lp, int n_seq, const int32_t* seqs, const uint8_t* masks);
 /* State of sequence `seq` after its bootstrap (host arrays): frame uint8 (rows,cols) tight at the sequence's own frame size
  * (b200vo_loop_set_frame_size) = the current frame;
  * lm float32 (n_lm,3) + lm_kp float32 (n_lm,2); keys / first_keys float32 (n_cand,2) + first_pose int32 (n_cand)

@@ -63,6 +63,9 @@ SIGNATURES = {
     "b200vo_good_features_to_track": (C.c_int, [
         C.c_void_p, c_u8p, C.c_int, C.c_int, C.c_size_t, C.c_int, C.c_double, C.c_double, C.c_int,
         c_f32p, c_intp]),
+    "b200vo_good_features_to_track_masked": (C.c_int, [
+        C.c_void_p, c_u8p, C.c_int, C.c_int, C.c_size_t, c_u8p, C.c_size_t, C.c_int, C.c_double, C.c_double, C.c_int,
+        c_f32p, c_intp]),
     "b200vo_knn2_ratio": (C.c_int, [
         C.c_void_p, c_f32p, C.c_int, c_f32p, C.c_int, C.c_int, C.c_double, c_i32p, c_f32p, c_u8p]),
     "b200vo_find_essential_mat_ransac": (C.c_int, [
@@ -86,6 +89,8 @@ SIGNATURES = {
     "b200vo_debug_pose_phases": (C.c_int, [
         C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, c_f64p, C.c_int, C.c_float, C.c_double, C.POINTER(C.c_longlong), c_f32p]),
     "b200vo_sift_detect_and_compute": (C.c_int, [C.c_void_p, c_u8p, C.c_int, C.c_int, C.c_size_t, C.c_int, c_f32p, c_f32p, c_i32p]),
+    "b200vo_sift_detect_and_compute_masked": (C.c_int, [C.c_void_p, c_u8p, C.c_int, C.c_int, C.c_size_t, c_u8p, C.c_size_t, C.c_int,
+                                                        c_f32p, c_f32p, c_i32p]),
     "b200vo_recover_pose": (C.c_int, [C.c_void_p, c_f64p, c_f32p, c_f32p, C.c_int, c_f64p, C.c_double, c_f64p, c_f64p, c_u8p, c_intp]),
     "b200vo_min_distance_mask": (C.c_int, [C.c_void_p, c_f32p, C.c_int, c_f32p, C.c_int, C.c_float, c_u8p]),
     "b200vo_triangulate_landmarks": (C.c_int, [
@@ -105,6 +110,7 @@ SIGNATURES = {
     "b200vo_batch_destroy": (None, [C.c_void_p]),
     "b200vo_batch_set_intrinsics": (C.c_int, [C.c_void_p, C.c_int, c_i32p, c_f64p]),
     "b200vo_batch_set_frame_size": (C.c_int, [C.c_void_p, C.c_int, c_i32p, c_i32p, c_i32p]),
+    "b200vo_batch_set_detection_mask": (C.c_int, [C.c_void_p, C.c_int, c_i32p, c_u8p]),
     "b200vo_batch_prime": (C.c_int, [C.c_void_p, c_u8p]),
     "b200vo_batch_submit_frames": (C.c_int, [C.c_void_p, c_u8p]),
     "b200vo_batch_submit_frames_dev": (C.c_int, [C.c_void_p, C.c_void_p]),
@@ -119,6 +125,7 @@ SIGNATURES = {
     "b200vo_loop_destroy": (None, [C.c_void_p]),
     "b200vo_loop_set_intrinsics": (C.c_int, [C.c_void_p, C.c_int, c_i32p, c_f64p]),
     "b200vo_loop_set_frame_size": (C.c_int, [C.c_void_p, C.c_int, c_i32p, c_i32p, c_i32p]),
+    "b200vo_loop_set_detection_mask": (C.c_int, [C.c_void_p, C.c_int, c_i32p, c_u8p]),
     "b200vo_loop_load": (C.c_int, [C.c_void_p, C.c_int, c_u8p, c_f32p, c_f32p, C.c_int, c_f32p, c_f32p, c_i32p, C.c_int, c_f64p,
                                    C.c_int]),
     "b200vo_loop_read_state": (C.c_int, [C.c_void_p, C.c_int, c_f32p, c_f32p, c_i32p, c_f32p, c_f32p, c_i32p, c_i32p, c_f64p, c_i32p,

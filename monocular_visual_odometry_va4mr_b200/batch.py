@@ -67,6 +67,29 @@ def _set_frame_size(ctx, fn, h, seqs, sizes, what):
     return seqs, np.stack([rows, cols], 1)
 
 
+def _set_detection_mask(ctx, fn, h, batch, frame_size, rows, cols, seqs, masks, what):
+    """Shared body of SequenceBatch / VOBatch.set_detection_mask.  -> the int32 seqs the call took."""
+    seqs = np.asarray(seqs)
+    if seqs.ndim != 1 or not 1 <= seqs.size <= batch or not np.issubdtype(seqs.dtype, np.integer):
+        raise ValueError(f"seqs must be 1 to batch = {batch} integer sequence indices, got {seqs.dtype} {seqs.shape}")
+    if ((seqs < 0) | (seqs >= batch)).any():
+        raise ValueError(f"seqs must lie in [0, batch = {batch})")
+    seqs = np.ascontiguousarray(seqs, np.int32)
+    if masks is not None:
+        if isinstance(masks, (list, tuple)):
+            masks = _pack_frames(list(masks), frame_size[seqs], rows, cols)
+        masks = np.asarray(masks)
+        if masks.dtype != np.uint8 or masks.shape != (len(seqs), rows, cols):
+            raise ValueError(f"masks must be ({len(seqs)}, {rows}, {cols}) uint8 or a list of {len(seqs)} masks, got {masks.dtype} {masks.shape}")
+        masks = np.ascontiguousarray(masks)
+    rc = fn(h, len(seqs), _p(seqs, c_i32p), None if masks is None else _p(masks, c_u8p))
+    if rc == -1:
+        raise ValueError(f"{what}: {ctx.last_error()}")
+    if rc != 0:
+        raise _lib.B200VOError(f"{what} failed ({rc}): {ctx.last_error()}")
+    return seqs
+
+
 def _pack_frames(frames, sizes, rows, cols, out=None):
     """A list of per-sequence 2-D uint8 images, each of its sequence's (rows_s, cols_s), packed into the slot layout
     (len, rows, cols); the bytes outside each image are zero.  An array is returned as it is."""
@@ -122,6 +145,7 @@ class SequenceBatch:
         self.batch, self.rows, self.cols = int(batch), int(rows), int(cols)
         self.L, self.Cn = int(max_landmarks), int(max_candidates)
         self.frame_size = np.tile(np.int32([self.rows, self.cols]), (self.batch, 1))   # (batch, 2) rows, cols of every sequence
+        self.has_mask = np.zeros(self.batch, bool)   # the sequences with a detection mask (set_detection_mask)
         self._submitted = []   # page-locked slot-layout copies of submitted frame lists, alive until their step
         cfg = BatchCfg()
         cfg.rows, cfg.cols = self.rows, self.cols
@@ -192,6 +216,18 @@ class SequenceBatch:
         Synchronous."""
         seqs, sizes = _set_frame_size(self.ctx, self.ctx.lib.b200vo_batch_set_frame_size, self.h, seqs, sizes, "b200vo_batch_set_frame_size")
         self.frame_size[seqs] = sizes
+        self.has_mask[seqs] = False
+
+    def set_detection_mask(self, seqs, masks):
+        """Give the distinct sequences ``seqs`` detection masks (cv2's ``goodFeaturesToTrack(..., mask=)``): ``masks`` is
+        (len(seqs), rows, cols) uint8 in the slot layout (a sequence's mask is the top-left of its row, at its frame size), or a
+        list of per-sequence 2-D uint8 masks at each sequence's frame size; None clears the listed sequences' masks.
+        ``good_features`` then detects in a masked sequence as ``cv2_compat.good_features_to_track_masked`` does on its frame.
+        ``set_frame_size`` clears the listed sequences' masks.  Bad shapes, dtypes or indices raise ValueError and change
+        nothing.  Synchronous."""
+        seqs = _set_detection_mask(self.ctx, self.ctx.lib.b200vo_batch_set_detection_mask, self.h, self.batch, self.frame_size,
+                                   self.rows, self.cols, seqs, masks, "b200vo_batch_set_detection_mask")
+        self.has_mask[seqs] = masks is not None
 
     def _frames(self, frames):
         """frames of a step: the slot-layout array, or a list of per-sequence 2-D images packed into it"""
@@ -322,6 +358,7 @@ class VOBatch:
         self.ctx = ctx or _lib.default_context(0)
         self.batch, self.rows, self.cols = int(batch), int(rows), int(cols)
         self.frame_size = np.tile(np.int32([self.rows, self.cols]), (self.batch, 1))   # (batch, 2) rows, cols of every sequence
+        self.has_mask = np.zeros(self.batch, bool)   # the sequences with a detection mask (set_detection_mask)
         self._submitted = []
         self.L, self.Cn, self.P = int(max_landmarks), int(max_candidates), int(max_frames)
         self.options = options
@@ -387,6 +424,19 @@ class VOBatch:
         still waiting, raise ValueError and change nothing.  Synchronous."""
         seqs, sizes = _set_frame_size(self.ctx, self.ctx.lib.b200vo_loop_set_frame_size, self.h, seqs, sizes, "b200vo_loop_set_frame_size")
         self.frame_size[seqs] = sizes
+        self.has_mask[seqs] = False
+
+    def set_detection_mask(self, seqs, masks):
+        """Give the distinct sequences ``seqs`` detection masks, for static regions whose corners move with the camera (a car's
+        hood, the black wedges of an undistorted image, a burned-in timestamp).  ``masks``: (len(seqs), rows, cols) uint8 in the
+        slot layout, or a list of per-sequence 2-D uint8 masks at each sequence's frame size; None clears the listed sequences'
+        masks.  A mask gates detection only: the corners a step adds (as ``cv2_compat.good_features_to_track_masked``) and
+        both SIFT frames of ``bootstrap`` (as ``match_bootstrap_frames(..., mask=)``); tracking, pose and triangulation do not
+        read it.  The sequences' states, status and frames are not touched; ``set_frame_size`` clears the listed sequences'
+        masks.  Bad shapes, dtypes or indices raise ValueError and change nothing.  Synchronous."""
+        seqs = _set_detection_mask(self.ctx, self.ctx.lib.b200vo_loop_set_detection_mask, self.h, self.batch, self.frame_size,
+                                   self.rows, self.cols, seqs, masks, "b200vo_loop_set_detection_mask")
+        self.has_mask[seqs] = masks is not None
 
     def load(self, seq: int, frame: np.ndarray, state: dict, K=None):
         """Set sequence ``seq`` to ``state`` (see the class docstring) with ``frame`` as its current frame; its status
@@ -551,16 +601,17 @@ class VOBatch:
                                                     o['pose_cw']), "b200vo_loop_step_dev")
 
 
-def match_bootstrap_frames(frame0, frame1, ratio=0.8):
+def match_bootstrap_frames(frame0, frame1, ratio=0.8, mask=None):
     """The reference's bootstrap matching (``VisualOdometryPipeLine.py:209-245``) on the CUDA path: SIFT
-    detectAndCompute on both frames, knnMatch(k=2) and the ratio test.  -> (pts0, pts1) float32 (n, 2)."""
+    detectAndCompute on both frames, knnMatch(k=2) and the ratio test.  -> (pts0, pts1) float32 (n, 2).
+    ``mask``: the detection mask of both SIFT calls (``cv2_compat.sift_detect_and_compute(..., mask=)``)."""
     from . import cv2_compat
-    sift = cv2_compat.SIFT_create()
-    kp0, d0 = sift.detectAndCompute(frame0, None)
-    kp1, d1 = sift.detectAndCompute(frame1, None)
-    good = [m for m, n in cv2_compat.BFMatcher().knnMatch(d0, d1, k=2) if m.distance < ratio * n.distance]
-    pts0 = np.float32([kp0[m.queryIdx].pt for m in good]).reshape(-1, 2)
-    pts1 = np.float32([kp1[m.trainIdx].pt for m in good]).reshape(-1, 2)
+    kp0, _, d0 = cv2_compat.sift_detect_and_compute(frame0, mask=mask)
+    kp1, _, d1 = cv2_compat.sift_detect_and_compute(frame1, mask=mask)
+    good = [m for m, n in cv2_compat.BFMatcher().knnMatch(d0 if len(d0) else None, d1 if len(d1) else None, k=2)
+            if m.distance < ratio * n.distance]
+    pts0 = np.float32([kp0[m.queryIdx, :2] for m in good]).reshape(-1, 2)
+    pts1 = np.float32([kp1[m.trainIdx, :2] for m in good]).reshape(-1, 2)
     return pts0, pts1
 
 

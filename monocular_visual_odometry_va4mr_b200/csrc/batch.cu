@@ -129,6 +129,7 @@ extern "C" int b200vo_batch_create(b200vo_ctx* ctx, int batch, const b200vo_batc
     for (int k = 1; k < batch; ++k) B->ext_host[k] = B->ext_host[0];
     rc = vo_reserve(ctx, B->ext_buf, (size_t)batch * sizeof(VoSeqExt));
     if (rc) { b200vo_batch_destroy(B); return rc; }
+    B->mask_host.assign(batch, 0);   // no masks (and no mask buffer until the first one)
     *out = B;
     return 0;
 }
@@ -182,7 +183,61 @@ int batch_set_frame_size(b200vo_batch* B, int n_seq, const int32_t* seqs, const 
     VO_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     B->ext_host.swap(ext);
     B->ext = uniform ? nullptr : (const VoSeqExt*)B->ext_buf.p;
+    // a mask has its sequence's frame size: the listed sequences lose theirs
+    bool had_mask = false;
+    for (int k = 0; k < n_seq; ++k) had_mask = had_mask || B->mask_host[seqs[k]];
+    if (had_mask) VO_TRY(batch_set_detection_mask(B, n_seq, seqs, nullptr));
     return 0;
+}
+
+int batch_set_detection_mask(b200vo_batch* B, int n_seq, const int32_t* seqs, const uint8_t* masks)
+{
+    b200vo_ctx* ctx = B->ctx;
+    const b200vo_batch_cfg& c = B->cfg;
+    if (n_seq < 1 || n_seq > B->batch) return vo_set_err(ctx, B200VO_E_BADARG, "n_seq = %d is outside [1, batch = %d]", n_seq, B->batch);
+    if (!seqs) return vo_set_err(ctx, B200VO_E_BADARG, "null array");
+    std::vector<char> seen(B->batch, 0);
+    for (int k = 0; k < n_seq; ++k) {
+        if (seqs[k] < 0 || seqs[k] >= B->batch)
+            return vo_set_err(ctx, B200VO_E_BADARG, "seqs[%d] = %d is outside [0, batch = %d)", k, seqs[k], B->batch);
+        if (seen[seqs[k]]++) return vo_set_err(ctx, B200VO_E_BADARG, "sequence %d is listed twice", seqs[k]);
+    }
+    const size_t fb = (size_t)c.rows * c.cols, b_on = vo_align((size_t)B->batch, 256);
+    std::vector<uint8_t> on = B->mask_host;
+    for (int k = 0; k < n_seq; ++k) on[seqs[k]] = masks ? 1 : 0;
+    VO_CUDA(ctx, cudaSetDevice(ctx->device));
+    VO_CUDA(ctx, cudaStreamSynchronize(ctx->stream));   // no step in flight reads the masks
+    VO_CUDA(ctx, cudaStreamSynchronize(B->pre_stream));
+    if (masks) VO_TRY(vo_reserve(ctx, B->mask_buf, b_on + B->batch * fb));
+    if (B->mask_buf.p) {
+        uint8_t* d = (uint8_t*)B->mask_buf.p;
+        if (masks)
+            for (int k = 0; k < n_seq; ++k)
+                VO_CUDA(ctx, cudaMemcpyAsync(d + b_on + seqs[k] * fb, masks + k * fb, fb, cudaMemcpyHostToDevice, ctx->stream));
+        VO_CUDA(ctx, cudaMemcpyAsync(d, on.data(), on.size(), cudaMemcpyHostToDevice, ctx->stream));
+        VO_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    }
+    B->mask_host.swap(on);
+    return 0;
+}
+
+VoMask batch_mask(const b200vo_batch* B)
+{
+    VoMask m;
+    bool any = false;
+    for (uint8_t f : B->mask_host) any = any || f;
+    if (!any) return m;
+    const uint8_t* d = (const uint8_t*)B->mask_buf.p;
+    m.on = d;
+    m.px = d + vo_align((size_t)B->batch, 256);
+    m.stride = (size_t)B->cfg.rows * B->cfg.cols;
+    m.pitch = B->cfg.cols;
+    return m;
+}
+
+extern "C" int b200vo_batch_set_detection_mask(b200vo_batch* B, int n_seq, const int32_t* seqs, const uint8_t* masks)
+{
+    return B ? batch_set_detection_mask(B, n_seq, seqs, masks) : B200VO_E_BADARG;
 }
 
 extern "C" int b200vo_batch_set_frame_size(b200vo_batch* B, int n_seq, const int32_t* seqs, const int32_t* rows, const int32_t* cols)
@@ -255,7 +310,8 @@ extern "C" void b200vo_batch_destroy(b200vo_batch* B)
     kill_stream(B->io_stream);
     kill_stream(B->pose_stream);
     for (auto& s : B->slabs) if (s.p) cudaFree(s.p);
-    for (DevBuf* d : {&B->raw, &B->raw_pre, &B->pts_in, &B->outs, &B->work, &B->gftt_ws, &B->intr_buf, &B->ext_buf, &B->lists})
+    for (DevBuf* d : {&B->raw, &B->raw_pre, &B->pts_in, &B->outs, &B->work, &B->gftt_ws, &B->intr_buf, &B->ext_buf, &B->lists,
+                     &B->mask_buf})
         if (d->p) cudaFree(d->p);
     for (auto& e : B->q_ev) kill_event(e);
     for (auto& e : B->chunk_ev) kill_event(e);
@@ -859,7 +915,7 @@ extern "C" int b200vo_batch_good_features(b200vo_batch* B, int max_corners, doub
     float* d_out = nullptr;
     int* d_small = nullptr;
     VO_TRY(vo_gftt_batch_launch(ctx, (const uint8_t*)B->slabs[B->cur].p + B->geom.off[0], B->geom.slab_bytes, B->geom.pitch[0], c.rows, c.cols,
-                                nb, max_corners, quality, min_dist, B->gftt_ws.p, &d_out, &d_small, B->ext));
+                                nb, max_corners, quality, min_dist, B->gftt_ws.p, &d_out, &d_small, B->ext, nullptr, 0, batch_mask(B)));
     const size_t b_out = vo_align((size_t)max_corners * 8, 256);
     const size_t out_bytes = b_out * nb, small_bytes = (size_t)nb * VO_GFTT_SMALL * sizeof(int);
     VO_TRY(vo_reserve_pinned(ctx, out_bytes + small_bytes));

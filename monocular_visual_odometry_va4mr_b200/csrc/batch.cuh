@@ -62,6 +62,10 @@ struct b200vo_batch {
     DevBuf ext_buf;
     const VoSeqExt* ext = nullptr;
     std::vector<VoSeqExt> ext_host;
+    // the detection mask of every sequence (b200vo_batch_set_detection_mask): [batch] "has a mask" bytes, then [batch] masks
+    // in the slot layout, allocated with the first mask.  mask_host mirrors the flags; no flag set: the detectors get no mask.
+    DevBuf mask_buf;
+    std::vector<uint8_t> mask_host;
     // host-input path: frames arrive chunk by chunk on a copy stream while earlier chunks are tracked
     cudaStream_t chunk_stream[B200VO_BATCH_STREAMS] = {};  // chunk k: H2D -> pyramid -> KLT on stream k % STREAMS
     cudaEvent_t chunk_ev[B200VO_BATCH_CHUNKS] = {};
@@ -101,6 +105,11 @@ int batch_set_intrinsics(b200vo_batch* B, int n_seq, const int32_t* seqs, const 
 // Validates the (index, rows, cols) triples and, only when all are valid and no submitted frame set waits, waits for the
 // work in flight and uploads the new extents (synchronous)
 int batch_set_frame_size(b200vo_batch* B, int n_seq, const int32_t* seqs, const int32_t* rows, const int32_t* cols);
+// Validates the n_seq distinct indices and, only when all are valid, waits for the work in flight and uploads the listed
+// sequences' masks (uint8 [n_seq][cfg.rows][cfg.cols]), or clears them (masks == nullptr).  Synchronous.
+int batch_set_detection_mask(b200vo_batch* B, int n_seq, const int32_t* seqs, const uint8_t* masks);
+// the masks of the detectors: indexed by sequence, none while no sequence has one
+VoMask batch_mask(const b200vo_batch* B);
 // the device rows of sequences [b0, ...) and their host copy, or nullptr for both while every sequence has the slot size
 inline const VoSeqExt* batch_ext_dev(const b200vo_batch* B, int b0) { return B->ext ? B->ext + b0 : nullptr; }
 inline const VoSeqExt* batch_ext_host(const b200vo_batch* B, int b0) { return B->ext ? B->ext_host.data() + b0 : nullptr; }

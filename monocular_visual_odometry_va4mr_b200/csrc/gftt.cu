@@ -157,11 +157,14 @@ gftt_colsum_kernel(const float* __restrict__ cov, int w, int h, float* __restric
 // forms the three covariance products of its column exactly as gftt_cov_kernel does, the double row sums come from
 // the neighbouring lanes by shuffle, and the three running column sums, the eigenvalue and the per-image maximum
 // follow -- the covariance and box planes (24 B per pixel) never exist in memory.
+// MASKED: an image with a mask leaves its maximum to gftt_mask_max_kernel.  Reading the mask here would put a load on
+// the serial chain of every row (or, prefetched, 30 more registers: two waves instead of one for 64 KITTI images).
 #define GF_COLS 30
+template <bool MASKED>
 __global__ void __launch_bounds__(32)
 gftt_fused_eig_kernel(const uint8_t* __restrict__ img, size_t img_stride, int pitch, int w, int h, float k0, float k1,
                       float* __restrict__ eig, int* __restrict__ max_bits, int small_stride, const VoSeqExt* __restrict__ ext,
-                      const int* __restrict__ list)
+                      const int* __restrict__ list, VoMask mk)
 {
     const int lane = threadIdx.x;
     const int im = list ? list[blockIdx.y] : blockIdx.y;
@@ -284,13 +287,46 @@ gftt_fused_eig_kernel(const uint8_t* __restrict__ img, size_t img_stride, int pi
     }
     cov_row(h, c);                                                   // last entering row: image row h-2
     emit(h - 1, c);
+    if (MASKED && (!mk.on || mk.on[im])) return;
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) vmax = fmaxf(vmax, __shfl_xor_sync(0xffffffffu, vmax, o));
     if (lane == 0 && vmax > __int_as_float(*(volatile int*)max_bits)) atomicMax(max_bits, __float_as_int(vmax));
 }
 
+// The maximum of each masked image's eigenvalue plane over the pixels of nonzero mask bytes, the 1-pixel border included
+// (cv2's minMaxLoc(eig, mask)), clamped at 0 as the unmasked maximum is: with a masked maximum <= 0 no masked pixel passes
+// `v > thr` anyway.  One CTA per 8 rows of an image; images without a mask return at once.
 __global__ void __launch_bounds__(256)
-gftt_eig_kernel(const float* __restrict__ box, int w, int h, float* __restrict__ eig, int* __restrict__ max_bits, int small_stride)
+gftt_mask_max_kernel(const float* __restrict__ eig, int w, int h, int* __restrict__ max_bits, int small_stride,
+                     const VoSeqExt* __restrict__ ext, const int* __restrict__ list, VoMask mk)
+{
+    const int im = list ? list[blockIdx.y] : blockIdx.y;
+    if (mk.on && !mk.on[im]) return;
+    eig += (size_t)im * w * h;                  // rows of the image's own width, as gftt_fused_eig_kernel writes them
+    if (ext) { w = ext[im].w[0]; h = ext[im].h[0]; }
+    const uint8_t* m = mk.px + im * mk.stride;
+    float vmax = 0.f;
+    for (int y = blockIdx.x * 8; y < min(h, (int)blockIdx.x * 8 + 8); ++y)
+        for (int x = threadIdx.x; x < w; x += blockDim.x)
+            if (m[(size_t)y * mk.pitch + x]) vmax = fmaxf(vmax, eig[(size_t)y * w + x]);
+    __shared__ float s_max[8];
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) vmax = fmaxf(vmax, __shfl_xor_sync(0xffffffffu, vmax, o));
+    if ((threadIdx.x & 31) == 0) s_max[threadIdx.x >> 5] = vmax;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        float mx = s_max[0];
+#pragma unroll
+        for (int k = 1; k < 8; ++k) mx = fmaxf(mx, s_max[k]);
+        max_bits += im * small_stride;
+        if (mx > __int_as_float(*(volatile int*)max_bits)) atomicMax(max_bits, __float_as_int(mx));
+    }
+}
+
+template <bool MASKED>
+__global__ void __launch_bounds__(256)
+gftt_eig_kernel(const float* __restrict__ box, int w, int h, float* __restrict__ eig, int* __restrict__ max_bits, int small_stride,
+                const uint8_t* __restrict__ mask /* MASKED: tight rows of w bytes */)
 {
     const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x, npx = (size_t)w * h;
     box += (size_t)blockIdx.y * 3 * npx;
@@ -307,6 +343,7 @@ gftt_eig_kernel(const float* __restrict__ box, int w, int h, float* __restrict__
     // One atomic per CTA, and only when it can raise the running maximum (a batch has 64 hot addresses).
     __shared__ float s_max[8];
     float vmax = fmaxf(v, 0.f);
+    if (MASKED && i < npx && !mask[i]) vmax = 0.f;           // the maximum over the masked pixels only (minMaxLoc(eig, mask))
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) vmax = fmaxf(vmax, __shfl_xor_sync(0xffffffffu, vmax, o));
     if ((threadIdx.x & 31) == 0) s_max[threadIdx.x >> 5] = vmax;
@@ -319,14 +356,17 @@ gftt_eig_kernel(const float* __restrict__ box, int w, int h, float* __restrict__
     }
 }
 
+// MASKED: a candidate also needs a nonzero mask byte at its pixel (the neighbours are compared whatever their mask)
+template <bool MASKED>
 __global__ void __launch_bounds__(256)
 gftt_candidates_kernel(const float* __restrict__ eig, int w, int h, const int* __restrict__ max_bits, double quality,
                        unsigned long long* __restrict__ keys, int* __restrict__ n_keys, int cap, int small_stride,
-                       const VoSeqExt* __restrict__ ext = nullptr, const int* __restrict__ list = nullptr)
+                       const VoSeqExt* __restrict__ ext, const int* __restrict__ list, VoMask mk)
 {
     const int im = list ? list[blockIdx.z] : blockIdx.z;
     eig += (size_t)im * w * h;
     if (ext) { w = ext[im].w[0]; h = ext[im].h[0]; }   // key address y * w + x: cv2's tie order in its own image
+    const uint8_t* mimg = MASKED && (!mk.on || mk.on[im]) ? mk.px + im * mk.stride : nullptr;
     max_bits += im * small_stride;
     n_keys += im * small_stride;
     keys += (size_t)im * cap;
@@ -340,8 +380,9 @@ gftt_candidates_kernel(const float* __restrict__ eig, int w, int h, const int* _
         float v = 0.f;
         if (x < w - 1 && y < h - 1) {
             const float* p = eig + (size_t)y * w + x;
+            const bool in_mask = !MASKED || !mimg || mimg[(size_t)y * mk.pitch + x] != 0;   // loaded beside the pixel
             v = p[0];
-            if (v > thr)
+            if (v > thr && in_mask)
                 is_c = !(p[-w - 1] > v || p[-w] > v || p[-w + 1] > v || p[-1] > v || p[1] > v || p[w - 1] > v || p[w] > v || p[w + 1] > v);
         }
         const unsigned m = __ballot_sync(0xffffffffu, is_c);
@@ -560,9 +601,9 @@ gftt_select_smem_kernel(const unsigned long long* __restrict__ sorted, const int
     if (lane == 0) *n_out = n_acc;
 }
 
-extern "C" int b200vo_good_features_to_track(b200vo_ctx* ctx, const uint8_t* img, int rows, int cols, size_t step,
-                                             int max_corners, double quality, double min_dist, int block_size,
-                                             float* corners_xy, int* n_out)
+// the host forms of goodFeaturesToTrack; mask: uint8 rows x cols, `mask_step` bytes a row, or nullptr
+static int gftt_host(b200vo_ctx* ctx, const uint8_t* img, int rows, int cols, size_t step, const uint8_t* mask, size_t mask_step,
+                     int max_corners, double quality, double min_dist, int block_size, float* corners_xy, int* n_out)
 {
     if (!ctx || !img || !corners_xy || !n_out) return B200VO_E_BADARG;
     *n_out = 0;
@@ -581,11 +622,20 @@ extern "C" int b200vo_good_features_to_track(b200vo_ctx* ctx, const uint8_t* img
     VO_TRY(vo_reserve(ctx, fs.slab, g.slab_bytes));
     fs.valid = false;
     VO_TRY(vo_reserve(ctx, ctx->d_stage_img[1], npx));
-    VO_TRY(vo_reserve_pinned(ctx, vo_align(npx, 256) + 4096));
+    VO_TRY(vo_reserve_pinned(ctx, vo_align(npx, 256) + 4096 + (mask ? npx : 0)));
     uint8_t* hp = (uint8_t*)ctx->h_pin;
     if (step == (size_t)cols) memcpy(hp, img, npx);
     else for (int y = 0; y < rows; ++y) memcpy(hp + (size_t)y * cols, img + (size_t)y * step, (size_t)cols);
     VO_CUDA(ctx, cudaMemcpyAsync(ctx->d_stage_img[1].p, hp, npx, cudaMemcpyHostToDevice, ctx->stream));
+    VoMask mk;   // tight rows of cols bytes on the device
+    if (mask) {
+        uint8_t* hm = hp + vo_align(npx, 256) + 4096;
+        for (int y = 0; y < rows; ++y) memcpy(hm + (size_t)y * cols, mask + (size_t)y * mask_step, (size_t)cols);
+        VO_TRY(vo_reserve(ctx, ctx->d_mask, npx));
+        VO_CUDA(ctx, cudaMemcpyAsync(ctx->d_mask.p, hm, npx, cudaMemcpyHostToDevice, ctx->stream));
+        mk.px = (const uint8_t*)ctx->d_mask.p;
+        mk.pitch = cols;
+    }
     VO_TRY(vo_build_pyramids(ctx, (const uint8_t*)ctx->d_stage_img[1].p, npx, rows, cols, g, (uint8_t*)fs.slab.p, g.slab_bytes, 1, ctx->stream));
     const uint8_t* d_img = (const uint8_t*)fs.slab.p + g.off[0];
     // scratch: cov | eig | keys | sorted | cells | small
@@ -619,11 +669,17 @@ extern "C" int b200vo_good_features_to_track(b200vo_ctx* ctx, const uint8_t* img
         gftt_cov_kernel<<<grd, blk, 0, ctx->stream>>>(d_img, 0, g.pitch[0], w, h, (float)scale, (float)(2.0 * scale), d_cov);
         gftt_rowsum_kernel<<<dim3((w + 255) / 256, h + 2), 256, 0, ctx->stream>>>(d_cov, w, h, d_rs);
         gftt_colsum_rs_kernel<<<(3 * w + 31) / 32, 32, 0, ctx->stream>>>(d_rs, w, h, d_box);
-        gftt_eig_kernel<<<(int)((npx + 255) / 256), 256, 0, ctx->stream>>>(d_box, w, h, d_eig, d_small, 0);
-        ctx->launches += 2;
         dim3 grd2((w - 2 + 31) / 32, (h - 2 + 31) / 32);
-        gftt_candidates_kernel<<<grd2, blk, 0, ctx->stream>>>(d_eig, w, h, d_small, quality, d_keys, d_small + 1, cap, 0);
-        ctx->launches += 3;
+        if (mk.px) {
+            gftt_eig_kernel<true><<<(int)((npx + 255) / 256), 256, 0, ctx->stream>>>(d_box, w, h, d_eig, d_small, 0, mk.px);
+            gftt_candidates_kernel<true><<<grd2, blk, 0, ctx->stream>>>(d_eig, w, h, d_small, quality, d_keys, d_small + 1, cap, 0,
+                                                                        nullptr, nullptr, mk);
+        } else {
+            gftt_eig_kernel<false><<<(int)((npx + 255) / 256), 256, 0, ctx->stream>>>(d_box, w, h, d_eig, d_small, 0, nullptr);
+            gftt_candidates_kernel<false><<<grd2, blk, 0, ctx->stream>>>(d_eig, w, h, d_small, quality, d_keys, d_small + 1, cap, 0,
+                                                                         nullptr, nullptr, mk);
+        }
+        ctx->launches += 5;
     }
     // the candidate count decides the sort; reading it back costs one small sync (the call is synchronous anyway)
     int* h_small = (int*)(hp + vo_align(npx, 256));
@@ -673,6 +729,24 @@ extern "C" int b200vo_good_features_to_track(b200vo_ctx* ctx, const uint8_t* img
     return 0;
 }
 
+extern "C" int b200vo_good_features_to_track(b200vo_ctx* ctx, const uint8_t* img, int rows, int cols, size_t step,
+                                             int max_corners, double quality, double min_dist, int block_size,
+                                             float* corners_xy, int* n_out)
+{
+    return gftt_host(ctx, img, rows, cols, step, nullptr, 0, max_corners, quality, min_dist, block_size, corners_xy, n_out);
+}
+
+extern "C" int b200vo_good_features_to_track_masked(b200vo_ctx* ctx, const uint8_t* img, int rows, int cols, size_t step,
+                                                    const uint8_t* mask, size_t mask_step, int max_corners, double quality,
+                                                    double min_dist, int block_size, float* corners_xy, int* n_out)
+{
+    if (mask && mask_step < (size_t)cols) {
+        if (n_out) *n_out = 0;
+        return ctx ? vo_set_err(ctx, B200VO_E_BADARG, "mask_step < cols") : B200VO_E_BADARG;
+    }
+    return gftt_host(ctx, img, rows, cols, step, mask, mask_step, max_corners, quality, min_dist, block_size, corners_xy, n_out);
+}
+
 // Batched detection on device-resident bordered level-0 images (one per sequence, `img_stride` bytes apart):
 // every kernel above with the image index in the grid, one selection CTA per image, no intermediate host
 // synchronisation (at most GFTT_BATCH_CAP candidates per image, ranked by counting).
@@ -689,7 +763,7 @@ size_t vo_gftt_batch_workspace(int rows, int cols, int batch, int max_corners)
 
 int vo_gftt_batch_launch(b200vo_ctx* ctx, const uint8_t* d_img0, size_t img_stride, int pitch, int rows, int cols, int batch,
                          int max_corners, double quality, double min_dist, void* ws, float** d_corners_out, int** d_small_out,
-                         const VoSeqExt* d_ext, const int* d_list, int n_img)
+                         const VoSeqExt* d_ext, const int* d_list, int n_img, const VoMask& mk)
 {
     const int w = cols, h = rows;
     if (!d_list) n_img = batch;
@@ -712,12 +786,20 @@ int vo_gftt_batch_launch(b200vo_ctx* ctx, const uint8_t* d_img0, size_t img_stri
     VO_CUDA(ctx, cudaMemsetAsync(d_small, 0, (size_t)batch * GFTT_SMALL * sizeof(int), ctx->stream));
     const double scale = 1.0 / (4.0 * 3 * 255.0);
     dim3 blk(32, 8);
-    gftt_fused_eig_kernel<<<dim3((w + GF_COLS - 1) / GF_COLS, n_img), 32, 0, ctx->stream>>>(d_img0, img_stride, pitch, w, h, (float)scale,
-                                                                                            (float)(2.0 * scale), d_eig, d_small, GFTT_SMALL, d_ext,
-                                                                                            d_list);
-    gftt_candidates_kernel<<<dim3((w - 2 + 31) / 32, (h - 2 + 31) / 32, n_img), blk, 0, ctx->stream>>>(d_eig, w, h, d_small, quality, d_keys,
-                                                                                                    d_small + 1, GFTT_BATCH_CAP, GFTT_SMALL, d_ext,
-                                                                                                    d_list);
+    const dim3 g_eig((w + GF_COLS - 1) / GF_COLS, n_img), g_cand((w - 2 + 31) / 32, (h - 2 + 31) / 32, n_img);
+    if (mk.px) {
+        gftt_fused_eig_kernel<true><<<g_eig, 32, 0, ctx->stream>>>(d_img0, img_stride, pitch, w, h, (float)scale, (float)(2.0 * scale), d_eig,
+                                                                   d_small, GFTT_SMALL, d_ext, d_list, mk);
+        gftt_mask_max_kernel<<<dim3((h + 7) / 8, n_img), 256, 0, ctx->stream>>>(d_eig, w, h, d_small, GFTT_SMALL, d_ext, d_list, mk);
+        ctx->launches++;
+        gftt_candidates_kernel<true><<<g_cand, blk, 0, ctx->stream>>>(d_eig, w, h, d_small, quality, d_keys, d_small + 1, GFTT_BATCH_CAP,
+                                                                      GFTT_SMALL, d_ext, d_list, mk);
+    } else {
+        gftt_fused_eig_kernel<false><<<g_eig, 32, 0, ctx->stream>>>(d_img0, img_stride, pitch, w, h, (float)scale, (float)(2.0 * scale), d_eig,
+                                                                    d_small, GFTT_SMALL, d_ext, d_list, mk);
+        gftt_candidates_kernel<false><<<g_cand, blk, 0, ctx->stream>>>(d_eig, w, h, d_small, quality, d_keys, d_small + 1, GFTT_BATCH_CAP,
+                                                                       GFTT_SMALL, d_ext, d_list, mk);
+    }
     gftt_rank_kernel<<<dim3(GFTT_BATCH_CAP / 256, n_img), 256, 0, ctx->stream>>>(d_keys, d_small + 1, GFTT_BATCH_CAP, d_sorted, GFTT_SMALL,
                                                                                  d_list);
     if (cell_smem > 48 * 1024)

@@ -39,6 +39,17 @@ struct VoSeqExt {
     int w[VO_MAX_LEVELS], h[VO_MAX_LEVELS];
 };
 
+// Detection masks (cv2's `mask=` of goodFeaturesToTrack and SIFT): image im's mask is the top-left of px + im * stride,
+// rows `pitch` bytes apart, read at the image's own extents; a pixel may hold a corner or keypoint only where its byte is
+// nonzero.  on[im] == 0: image im has no mask (detected everywhere); on == nullptr: every image has one.  px == nullptr:
+// no image of the launch has a mask, and the detectors run exactly as without this argument.
+struct VoMask {
+    const uint8_t* px = nullptr;
+    const uint8_t* on = nullptr;
+    size_t stride = 0;
+    int pitch = 0;
+};
+
 struct KltParams {
     int win_w, win_h;
     int max_count;
@@ -103,6 +114,7 @@ struct b200vo_ctx {
     DevBuf d_rng;            // raw cv::RNG stream (uint32)
     int n_rng = 0;
     DevBuf d_intr;           // the one-row intrinsics array of the one-call entry points (vo_intrinsics_one)
+    DevBuf d_mask;           // the detection mask of the masked one-call entry points
     // tensor-map encode entry point (driver API, fetched lazily)
     void* encode_tiled = nullptr;
 };
@@ -180,10 +192,11 @@ int vo_build_pyramids(b200vo_ctx* ctx, const uint8_t* d_raw, size_t raw_stride, 
 #define VO_GFTT_BATCH_CAP 32768  // candidates per image the batched path can rank
 size_t vo_gftt_batch_workspace(int rows, int cols, int batch, int max_corners);
 // d_ext: [batch] per-sequence extents (level 0 is read), nullptr: every image is rows x cols.  d_list: only the n_img
-// images list[k] are detected; their outputs keep the image index (the others' are left stale)
+// images list[k] are detected; their outputs keep the image index (the others' are left stale).  mask: the images'
+// detection masks, indexed by the image index (no mask: the kernels without mask reads run)
 int vo_gftt_batch_launch(b200vo_ctx* ctx, const uint8_t* d_img0, size_t img_stride, int pitch, int rows, int cols, int batch,
                          int max_corners, double quality, double min_dist, void* ws, float** d_corners_out, int** d_small_out,
-                         const VoSeqExt* d_ext = nullptr, const int* d_list = nullptr, int n_img = 0);
+                         const VoSeqExt* d_ext = nullptr, const int* d_list = nullptr, int n_img = 0, const VoMask& mask = VoMask{});
 
 // ---- klt.cu ----
 struct KltPointSet {

@@ -332,7 +332,7 @@ static int loop_core(b200vo_loop* lp, const uint8_t* frames_dev, const LoopOut& 
     int* small = nullptr;
     VO_TRY(vo_gftt_batch_launch(ctx, (const uint8_t*)B->slabs[B->nxt].p + B->geom.off[0], B->geom.slab_bytes, B->geom.pitch[0],
                                 c.batch.rows, c.batch.cols, nb, c.max_corners, c.quality_level, c.feature_min_dist, B->gftt_ws.p,
-                                &corners, &small, B->ext, d.list, n_cta));
+                                &corners, &small, B->ext, d.list, n_cta, batch_mask(B)));
     d.corners = corners; d.gftt_small = small;
     loop_commit_kernel<<<n_cta, LOOP_T, 0, ctx->stream>>>(d, o);
     ctx->launches++;
@@ -596,6 +596,11 @@ extern "C" int b200vo_loop_set_frame_size(b200vo_loop* lp, int n_seq, const int3
     return 0;
 }
 
+extern "C" int b200vo_loop_set_detection_mask(b200vo_loop* lp, int n_seq, const int32_t* seqs, const uint8_t* masks)
+{
+    return lp ? batch_set_detection_mask(lp->B, n_seq, seqs, masks) : B200VO_E_BADARG;
+}
+
 extern "C" int b200vo_loop_read_state(b200vo_loop* lp, int seq, float* lm, float* lm_kp, int32_t* n_lm, float* keys, float* first_keys,
                                       int32_t* first_pose, int32_t* n_cand, double* poses, int32_t* n_poses, int32_t* status)
 {
@@ -780,11 +785,20 @@ extern "C" int b200vo_loop_bootstrap(b200vo_loop* lp, int n_seq, const int32_t* 
     VO_CUDA(ctx, cudaStreamSynchronize(ctx->stream));   // no step in flight reads the state
     cudaStream_t st = ctx->stream;
     // the two frames of sequence j of the run are frames 2j and 2j + 1 of the SIFT batch (slot layout)
-    const size_t b_raw = vo_align(ns * 2 * fb, 256), b_cnt = vo_align(ns * 8, 256);
-    VO_TRY(vo_reserve(ctx, lp->boot_in, b_raw + 2 * b_cnt));
+    const size_t b_raw = vo_align(ns * 2 * fb, 256), b_cnt = vo_align(ns * 8, 256), b_moff = vo_align(ns * 16, 256);
+    VO_TRY(vo_reserve(ctx, lp->boot_in, b_raw + 2 * b_cnt + b_moff));
     uint8_t* raw = (uint8_t*)lp->boot_in.p;
     int* d_nkp = (int*)(raw + b_raw);
     int* d_row = (int*)(raw + b_raw + b_cnt);
+    // both SIFT frames of a sequence with a detection mask use it: the offsets of the run's frames in the mask slab
+    const VoMask mk = batch_mask(B);
+    long long* d_moff = nullptr;
+    if (mk.px) {
+        std::vector<long long> moff(2 * ns);
+        for (int j = 0; j < n_seq; ++j) moff[2 * j] = moff[2 * j + 1] = B->mask_host[seqs[j]] ? (long long)(seqs[j] * mk.stride) : -1;
+        d_moff = (long long*)(raw + b_raw + 2 * b_cnt);
+        VO_CUDA(ctx, cudaMemcpyAsync(d_moff, moff.data(), ns * 16, cudaMemcpyHostToDevice, st));
+    }
     if (in_order) {
         VO_CUDA(ctx, cudaMemcpy2DAsync(raw, 2 * fb, frames0, fb, fb, ns, cudaMemcpyHostToDevice, st));
         VO_CUDA(ctx, cudaMemcpy2DAsync(raw + fb, 2 * fb, frames1, fb, fb, ns, cudaMemcpyHostToDevice, st));
@@ -800,7 +814,7 @@ extern "C" int b200vo_loop_bootstrap(b200vo_loop* lp, int n_seq, const int32_t* 
         const VoSeqExt& e = B->ext_host[seqs[j0]];
         const int m = grp_end[g] - (int)j0;
         VO_TRY(vo_sift_frames(ctx, raw + 2 * j0 * fb, fb, 2 * m, e.h[0], e.w[0], true, d_nkp + 2 * j0, d_row + 2 * j0, &n_rows, n_rows,
-                              (size_t)cols));
+                              (size_t)cols, mk.px, d_moff ? d_moff + 2 * j0 : nullptr));
     }
     std::vector<int> h_cnt(4 * ns);
     VO_CUDA(ctx, cudaMemcpyAsync(h_cnt.data(), d_nkp, ns * 8, cudaMemcpyDeviceToHost, st));

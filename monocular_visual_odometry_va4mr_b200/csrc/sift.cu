@@ -530,12 +530,17 @@ struct SiftKpLess {
 // order (cta_compact) at out[lo + rank]; the rest of the run is marked free.  Writes the kept keypoints in the
 // caller's format (firstOctave = -1 undone: coordinates and size halved, octave - 1 in the low byte) at kp6[base + lo + rank],
 // and per frame the count and the first row.
+// Detection mask (mask_off != nullptr): frame f's mask is at mask + mask_off[f] (rows `mask_pitch` bytes apart; < 0: none).
+// A keypoint whose byte at ((int)(y + 0.5f), (int)(x + 0.5f)) of the halved coordinates is 0 is dropped as well, as cv2's
+// KeyPointsFilter::runByPixelsMask drops it after the duplicates; duplicates share (x, y), so the two filters commute.
 __global__ void __launch_bounds__(SIFT_DEDUP_T)
 sift_dedup_kernel(const SiftKp* __restrict__ sorted, int n, SiftKp* __restrict__ out, float* __restrict__ kp6, int base,
-                  int* __restrict__ n_frame, int* __restrict__ first_row)
+                  int* __restrict__ n_frame, int* __restrict__ first_row, const uint8_t* __restrict__ mask,
+                  const long long* __restrict__ mask_off, int mask_pitch)
 {
     __shared__ int s_lo, s_hi;
     const int f = blockIdx.x;
+    const uint8_t* fm = mask_off && mask_off[f] >= 0 ? mask + mask_off[f] : nullptr;
     if (threadIdx.x < 2) {   // lower bounds of f and f + 1
         const int key = f + threadIdx.x;
         int a = 0, b = n;
@@ -545,9 +550,13 @@ sift_dedup_kernel(const SiftKp* __restrict__ sorted, int n, SiftKp* __restrict__
     __syncthreads();
     const int lo = s_lo, hi = s_hi;
     const int cnt = cta_compact<SIFT_DEDUP_T>(hi - lo, [&](int j) {
+        const SiftKp& k = sorted[lo + j];
+        if (fm) {
+            const int mx = (int)__fadd_rn(__fmul_rn(k.x, 0.5f), 0.5f), my = (int)__fadd_rn(__fmul_rn(k.y, 0.5f), 0.5f);
+            if (!fm[(size_t)my * mask_pitch + mx]) return false;
+        }
         if (j == 0) return true;
         const SiftKp& p = sorted[lo + j - 1];
-        const SiftKp& k = sorted[lo + j];
         return p.x != k.x || p.y != k.y || p.size != k.size || p.angle != k.angle;
     }, [&](int j, int o) {
         const SiftKp k = sorted[lo + j];
@@ -649,7 +658,8 @@ static int sift_reserve_keep(b200vo_ctx* ctx, DevBuf& b, size_t used, size_t byt
 }
 
 int vo_sift_frames(b200vo_ctx* ctx, const uint8_t* d_raw, size_t raw_stride, int n_frames, int rows, int cols, bool want_desc,
-                   int* d_n_frame, int* d_first_row, int* n_rows, int row0, size_t row_stride)
+                   int* d_n_frame, int* d_first_row, int* n_rows, int row0, size_t row_stride, const uint8_t* d_mask,
+                   const long long* d_mask_off)
 {
     const int L = SIFT_LAYERS;
     if (!row_stride) row_stride = (size_t)cols;
@@ -743,7 +753,8 @@ int vo_sift_frames(b200vo_ctx* ctx, const uint8_t* d_raw, size_t raw_stride, int
             ctx->launches += 1 + 2 * passes;
         }
         sift_dedup_kernel<<<nf, SIFT_DEDUP_T, 0, ctx->stream>>>(sorted, n_kp, kps, (float*)ctx->d_sift_out[0].p, base, d_n_frame + f0,
-                                                              d_first_row + f0);
+                                                              d_first_row + f0, d_mask, d_mask_off ? d_mask_off + f0 : nullptr,
+                                                              (int)row_stride);
         ctx->launches++;
         if (n_kp > 0 && want_desc) {
             sift_descriptor_kernel<<<n_kp, SIFT_DESC_T, 0, ctx->stream>>>(P, kps, n_kp, (float*)ctx->d_sift_out[1].p + (size_t)base * 128);
@@ -756,10 +767,12 @@ int vo_sift_frames(b200vo_ctx* ctx, const uint8_t* d_raw, size_t raw_stride, int
     return 0;
 }
 
-extern "C" int b200vo_sift_detect_and_compute(b200vo_ctx* ctx, const uint8_t* img, int rows, int cols, size_t step, int max_kp,
-                                              float* kps_out, float* desc_out, int32_t* n_out)
+// the host forms of SIFT detectAndCompute; mask: uint8 rows x cols, `mask_step` bytes a row, or nullptr
+static int sift_host(b200vo_ctx* ctx, const uint8_t* img, int rows, int cols, size_t step, const uint8_t* mask, size_t mask_step,
+                     int max_kp, float* kps_out, float* desc_out, int32_t* n_out)
 {
-    if (!ctx || !img || !n_out || rows <= 0 || cols <= 0 || step < (size_t)cols || max_kp < 0 || (max_kp > 0 && !kps_out))
+    if (!ctx || !img || !n_out || rows <= 0 || cols <= 0 || step < (size_t)cols || max_kp < 0 || (max_kp > 0 && !kps_out) ||
+        (mask && mask_step < (size_t)cols))
         return B200VO_E_BADARG;
     *n_out = 0;
     VO_CUDA(ctx, cudaSetDevice(ctx->device));
@@ -769,8 +782,20 @@ extern "C" int b200vo_sift_detect_and_compute(b200vo_ctx* ctx, const uint8_t* im
     uint8_t* raw = (uint8_t*)ctx->d_stage_img[0].p;
     int* d_small = (int*)(raw + vo_align((size_t)rows * cols, 128));   // count | first row
     VO_CUDA(ctx, cudaMemcpy2DAsync(raw, cols, img, step, cols, rows, cudaMemcpyHostToDevice, ctx->stream));
+    // the mask (tight rows, as the frame) after the one-entry table of its offset
+    const long long* d_moff = nullptr;
+    const uint8_t* d_mask = nullptr;
+    if (mask) {
+        VO_TRY(vo_reserve(ctx, ctx->d_mask, 256 + (size_t)rows * cols));
+        const long long zero = 0;
+        d_moff = (const long long*)ctx->d_mask.p;
+        d_mask = (const uint8_t*)ctx->d_mask.p + 256;
+        VO_CUDA(ctx, cudaMemcpyAsync(ctx->d_mask.p, &zero, sizeof(zero), cudaMemcpyHostToDevice, ctx->stream));
+        VO_CUDA(ctx, cudaMemcpy2DAsync((uint8_t*)ctx->d_mask.p + 256, cols, mask, mask_step, cols, rows, cudaMemcpyHostToDevice, ctx->stream));
+    }
     int n_rows = 0;
-    VO_TRY(vo_sift_frames(ctx, raw, (size_t)rows * cols, 1, rows, cols, desc_out != nullptr, d_small, d_small + 1, &n_rows));
+    VO_TRY(vo_sift_frames(ctx, raw, (size_t)rows * cols, 1, rows, cols, desc_out != nullptr, d_small, d_small + 1, &n_rows, 0, 0, d_mask,
+                          d_moff));
     // rows [0, count) of the outputs are the keypoints in cv2's order
     const size_t b_k = vo_align((size_t)n_rows * 24, 256), b_d = desc_out ? (size_t)n_rows * 512 : 0;
     VO_TRY(vo_reserve_pinned(ctx, 256 + b_k + b_d));
@@ -791,4 +816,17 @@ extern "C" int b200vo_sift_detect_and_compute(b200vo_ctx* ctx, const uint8_t* im
     }
     *n_out = cnt;
     return 0;
+}
+
+extern "C" int b200vo_sift_detect_and_compute(b200vo_ctx* ctx, const uint8_t* img, int rows, int cols, size_t step, int max_kp,
+                                              float* kps_out, float* desc_out, int32_t* n_out)
+{
+    return sift_host(ctx, img, rows, cols, step, nullptr, 0, max_kp, kps_out, desc_out, n_out);
+}
+
+extern "C" int b200vo_sift_detect_and_compute_masked(b200vo_ctx* ctx, const uint8_t* img, int rows, int cols, size_t step,
+                                                     const uint8_t* mask, size_t mask_step, int max_kp, float* kps_out,
+                                                     float* desc_out, int32_t* n_out)
+{
+    return sift_host(ctx, img, rows, cols, step, mask, mask_step, max_kp, kps_out, desc_out, n_out);
 }

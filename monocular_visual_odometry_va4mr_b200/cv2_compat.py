@@ -183,6 +183,39 @@ def goodFeaturesToTrack(image, maxCorners, qualityLevel, minDistance, corners=No
     return buf[:n_out.value].reshape(-1, 1, 2).copy()
 
 
+def _mask_arg(mask, shape, what):
+    """A detection mask: 2-D uint8 of the image's shape (cv2 raises cv2.error otherwise)."""
+    if not isinstance(mask, np.ndarray) or mask.dtype != np.uint8 or mask.shape != shape:
+        got = f"{mask.dtype} {mask.shape}" if isinstance(mask, np.ndarray) else type(mask).__name__
+        raise error(f"b200vo {what}: (-215:Assertion failed) mask.empty() || (mask.type() == CV_8UC1 && mask.sameSize(image)): "
+                    f"the mask must be uint8 {shape}, got {got}")
+    return np.ascontiguousarray(mask)
+
+
+def good_features_to_track_masked(image, maxCorners, qualityLevel, minDistance, mask, blockSize=3):
+    """cv2.goodFeaturesToTrack(image, maxCorners, qualityLevel, minDistance, mask=mask, blockSize=blockSize) -> float32 (M,1,2)
+    or None.  A corner needs a nonzero mask byte at its pixel, and the quality threshold is taken over the masked pixels
+    only, as cv2 does.  mask=None: the unmasked call.  A mask that is not uint8 of the image's shape raises ``error``."""
+    image, step = _image_arg(image, "image")
+    if mask is not None:
+        mask = _mask_arg(mask, image.shape, "goodFeaturesToTrack")
+    if not (qualityLevel > 0 and minDistance >= 0 and maxCorners >= 0):
+        raise error("b200vo goodFeaturesToTrack: (-215:Assertion failed) qualityLevel > 0 && minDistance >= 0 && maxCorners >= 0")
+    ctx = _ctx()
+    cap = int(maxCorners) if maxCorners > 0 else image.shape[0] * image.shape[1]
+    buf = np.empty((max(cap, 1), 2), np.float32)
+    n_out = C.c_int(0)
+    rc = ctx.lib.b200vo_good_features_to_track_masked(ctx.h, _p(image, c_u8p), image.shape[0], image.shape[1], step,
+                                                      None if mask is None else _p(mask, c_u8p), 0 if mask is None else mask.shape[1],
+                                                      int(maxCorners), float(qualityLevel), float(minDistance), int(blockSize),
+                                                      _p(buf, c_f32p), C.byref(n_out))
+    if rc != 0:
+        _raise(ctx, rc, "goodFeaturesToTrack")
+    if n_out.value == 0:
+        return None
+    return buf[:n_out.value].reshape(-1, 1, 2).copy()
+
+
 # --------------------------------------------------------------------------------------
 # cv2.BFMatcher().knnMatch + ratio test  (reference :36, :229, :218-224)
 # --------------------------------------------------------------------------------------
@@ -258,10 +291,14 @@ class KeyPoint:
         return f"KeyPoint(pt={self.pt}, size={self.size}, angle={self.angle}, octave={self.octave})"
 
 
-def sift_detect_and_compute(image, max_keypoints=1 << 17):
+def sift_detect_and_compute(image, max_keypoints=1 << 17, mask=None):
     """Array form: (kp float32 (n, 5) = x, y, size, angle, response; octave int32 (n,); descriptors float32 (n, 128)),
-    rows in cv2's output order."""
+    rows in cv2's output order.  ``mask``: cv2's detectAndCompute(image, mask), uint8 of the image's shape; a keypoint is
+    dropped where the byte at its rounded position is 0, the others keep their order and descriptors.  Unlike cv2, which
+    does not check it, a mask of another shape or dtype raises ``error``."""
     img, step = _image_arg(image, "SIFT.detectAndCompute image")
+    if mask is not None:
+        mask = _mask_arg(mask, img.shape, "SIFT.detectAndCompute")
     ctx = _ctx()
     rows, cols = img.shape
     cap = 8192
@@ -269,7 +306,12 @@ def sift_detect_and_compute(image, max_keypoints=1 << 17):
         kps = np.empty((cap, 6), np.float32)
         desc = np.empty((cap, 128), np.float32)
         n = C.c_int32(0)
-        rc = ctx.lib.b200vo_sift_detect_and_compute(ctx.h, _p(img, c_u8p), rows, cols, step, cap, _p(kps, c_f32p), _p(desc, c_f32p), C.byref(n))
+        if mask is None:
+            rc = ctx.lib.b200vo_sift_detect_and_compute(ctx.h, _p(img, c_u8p), rows, cols, step, cap, _p(kps, c_f32p), _p(desc, c_f32p),
+                                                        C.byref(n))
+        else:
+            rc = ctx.lib.b200vo_sift_detect_and_compute_masked(ctx.h, _p(img, c_u8p), rows, cols, step, _p(mask, c_u8p), cols, cap,
+                                                               _p(kps, c_f32p), _p(desc, c_f32p), C.byref(n))
         if rc != 0:
             _raise(ctx, rc, "SIFT.detectAndCompute")
         if n.value <= cap or cap >= max_keypoints:
