@@ -232,6 +232,15 @@ int b200vo_sift_detect_and_compute(b200vo_ctx* ctx, const uint8_t* img, int rows
 int b200vo_sift_detect_and_compute_masked(b200vo_ctx* ctx, const uint8_t* img, int rows, int cols, size_t step,
                                           const uint8_t* mask, size_t mask_step, int max_kp, float* kps,
                                           float* desc, int32_t* n_out);
+/*
+ * Replaces cv2.undistort(src, K, dist) (newCameraMatrix = K): src uint8 (rows, cols), `step` bytes a row; dst uint8
+ * (rows, cols), tight.  K a pinhole camera matrix (as b200vo_batch_set_intrinsics accepts); dist double [n_dist], n_dist
+ * 4 (k1, k2, p1, p2), 5 (+ k3) or 8 (+ k4, k5, k6, the rational model), all finite.  Byte for byte what cv2 computes: the
+ * map of initUndistortRectifyMap(..., CV_16SC2) (1/32 px) and a fixed-point bilinear remap with BORDER_CONSTANT 0, so
+ * pixels that map outside the image (or to a non-finite point) are 0.  Other n_dist: B200VO_E_UNSUPPORTED.
+ */
+int b200vo_undistort(b200vo_ctx* ctx, const uint8_t* src, int rows, int cols, size_t step, const double K[9],
+                     const double* dist, int n_dist, uint8_t* dst);
 
 /*
  * Replaces cv2.solvePnPRansac(obj, img, K, zeros(4), flags=SOLVEPNP_P3P, confidence=,
@@ -307,6 +316,20 @@ int b200vo_batch_set_frame_size(b200vo_batch* b, int n_seq, const int32_t* seqs,
  * steps included, as the frames' pyramids do not depend on it.
  */
 int b200vo_batch_set_detection_mask(b200vo_batch* b, int n_seq, const int32_t* seqs, const uint8_t* masks);
+/*
+ * Per-sequence lens distortion.  dist: double [n_seq][8], k1, k2, p1, p2, k3, k4, k5, k6 (cv2's order; pad shorter models
+ * with zeros); an all-zero row clears a sequence's distortion.  Every frame handed to the batch is raw camera output: a
+ * sequence with distortion has its level 0 built from cv2.undistort(frame, K, dist) (b200vo_undistort, newCameraMatrix =
+ * K), gathered on the device while the pyramid is built, so points, poses and detection masks are all in the undistorted
+ * image, whose camera is the sequence's K.  The map is a function of K, the coefficients and the frame size: this call,
+ * b200vo_batch_set_intrinsics and b200vo_batch_set_frame_size rebuild it for the sequences with distortion (the
+ * coefficients survive a frame-size change).  Bad indices (out of range, repeated), n_seq < 1, null arrays, a non-finite
+ * coefficient or submitted frame sets still waiting: B200VO_E_BADARG and nothing changes.  The resident frames no longer
+ * match: the next step needs b200vo_batch_prime.  While submitted frame sets wait, b200vo_batch_set_intrinsics refuses a
+ * sequence with distortion too.  The map memory (6 bytes a slot pixel per sequence) is allocated with the first
+ * distortion; a batch without distortion builds its pyramids as it always did.  Synchronous.
+ */
+int b200vo_batch_set_distortion(b200vo_batch* b, int n_seq, const int32_t* seqs, const double* dist);
 /* Upload the first frame of every sequence (frames: batch x rows x cols, tight). */
 int b200vo_batch_prime(b200vo_batch* b, const uint8_t* frames);
 /*
@@ -405,6 +428,12 @@ int b200vo_loop_set_frame_size(b200vo_loop* lp, int n_seq, const int32_t* seqs, 
  * results are those of the per-call masked forms on its frames; tracking, pose and triangulation do not read it.  The
  * state, status and frames are not touched.  Synchronous. */
 int b200vo_loop_set_detection_mask(b200vo_loop* lp, int n_seq, const int32_t* seqs, const uint8_t* masks);
+/* Per-sequence lens distortion of the loop, as b200vo_batch_set_distortion (same layout and validation: B200VO_E_BADARG,
+ * nothing changes).  Every frame the loop takes (steps, submitted sets, b200vo_loop_load, both frames of
+ * b200vo_loop_bootstrap) is raw camera output, undistorted on the device with the sequence's K before anything reads it;
+ * the loaded state, keypoints, landmarks, poses, b200vo_loop_read_state and detection masks are in the undistorted image.
+ * The listed sequences become B200VO_LOOP_IDLE until b200vo_loop_load or b200vo_loop_bootstrap runs for them.  Synchronous. */
+int b200vo_loop_set_distortion(b200vo_loop* lp, int n_seq, const int32_t* seqs, const double* dist);
 /* State of sequence `seq` after its bootstrap (host arrays): frame uint8 (rows,cols) tight at the sequence's own frame size
  * (b200vo_loop_set_frame_size) = the current frame;
  * lm float32 (n_lm,3) + lm_kp float32 (n_lm,2); keys / first_keys float32 (n_cand,2) + first_pose int32 (n_cand)

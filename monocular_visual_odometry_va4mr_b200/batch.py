@@ -90,6 +90,28 @@ def _set_detection_mask(ctx, fn, h, batch, frame_size, rows, cols, seqs, masks, 
     return seqs
 
 
+def _set_distortion(ctx, fn, h, batch, seqs, dist, what):
+    """Shared body of SequenceBatch / VOBatch.set_distortion.  -> (seqs, dist (len(seqs), 8)) as the call took them."""
+    seqs = np.asarray(seqs)
+    if seqs.ndim != 1 or not 1 <= seqs.size <= batch or not np.issubdtype(seqs.dtype, np.integer):
+        raise ValueError(f"seqs must be 1 to batch = {batch} integer sequence indices, got {seqs.dtype} {seqs.shape}")
+    seqs = np.ascontiguousarray(seqs, np.int32)
+    d8 = np.zeros((len(seqs), 8), np.float64)
+    if dist is not None:
+        d = np.asarray(dist)
+        if d.ndim == 2 and d.shape[0] == len(seqs) and d.shape[1] in (12, 14):
+            raise NotImplementedError("the thin-prism (12) and tilted (14) distortion models are not supported")
+        if d.ndim != 2 or d.shape[0] != len(seqs) or d.shape[1] not in (4, 5, 8) or not np.issubdtype(d.dtype, np.number):
+            raise ValueError(f"dist must be (len(seqs) = {len(seqs)}, 4 | 5 | 8) coefficients or None, got {d.dtype} {d.shape}")
+        d8[:, :d.shape[1]] = d
+    rc = fn(h, len(seqs), _p(seqs, c_i32p), _p(d8, c_f64p))
+    if rc == -1:
+        raise ValueError(f"{what}: {ctx.last_error()}")
+    if rc != 0:
+        raise _lib.B200VOError(f"{what} failed ({rc}): {ctx.last_error()}")
+    return seqs, d8
+
+
 def _pack_frames(frames, sizes, rows, cols, out=None):
     """A list of per-sequence 2-D uint8 images, each of its sequence's (rows_s, cols_s), packed into the slot layout
     (len, rows, cols); the bytes outside each image are zero.  An array is returned as it is."""
@@ -140,12 +162,13 @@ class _PinnedBlock:
 class SequenceBatch:
     def __init__(self, batch, rows, cols, K, win=(15, 15), max_level=5, criteria=(3, 50, 0.01),
                  min_eig_thr=1e-4, pnp_iters=500, pnp_reproj_err=8.0, pnp_conf=0.99,
-                 max_landmarks=1024, max_candidates=1024, frame_size=None, ctx: _lib.Context | None = None):
+                 max_landmarks=1024, max_candidates=1024, frame_size=None, dist_coeffs=None, ctx: _lib.Context | None = None):
         self.ctx = ctx or _lib.default_context(0)
         self.batch, self.rows, self.cols = int(batch), int(rows), int(cols)
         self.L, self.Cn = int(max_landmarks), int(max_candidates)
         self.frame_size = np.tile(np.int32([self.rows, self.cols]), (self.batch, 1))   # (batch, 2) rows, cols of every sequence
         self.has_mask = np.zeros(self.batch, bool)   # the sequences with a detection mask (set_detection_mask)
+        self.dist_coeffs = np.zeros((self.batch, 8))   # k1, k2, p1, p2, k3, k4, k5, k6 of every sequence (set_distortion)
         self._submitted = []   # page-locked slot-layout copies of submitted frame lists, alive until their step
         cfg = BatchCfg()
         cfg.rows, cfg.cols = self.rows, self.cols
@@ -168,6 +191,8 @@ class SequenceBatch:
             self.set_intrinsics(np.arange(self.batch), K_rows)
         if frame_size is not None:
             self.set_frame_size(np.arange(self.batch), frame_size)
+        if dist_coeffs is not None:
+            self.set_distortion(np.arange(self.batch), dist_coeffs)
         # host outputs (reused, page-locked so that step() reads them back without a staging copy)
         b, L, Cn = self.batch, self.L, self.Cn
         self.lm_next = self.pinned_empty((b, L, 2), np.float32)
@@ -228,6 +253,19 @@ class SequenceBatch:
         seqs = _set_detection_mask(self.ctx, self.ctx.lib.b200vo_batch_set_detection_mask, self.h, self.batch, self.frame_size,
                                    self.rows, self.cols, seqs, masks, "b200vo_batch_set_detection_mask")
         self.has_mask[seqs] = masks is not None
+
+    def set_distortion(self, seqs, dist):
+        """Give the distinct sequences ``seqs`` lens distortion: ``dist`` (len(seqs), n) with n = 4, 5 or 8 coefficients in cv2's
+        order (k1, k2, p1, p2[, k3[, k4, k5, k6]]), or None to clear it; an all-zero row clears it too.  Every frame of a
+        sequence with distortion is raw camera output that the batch undistorts on the device as ``cv2.undistort(frame, K,
+        dist)`` does (``cv2_compat.undistort``) before anything reads it: points, poses, ``good_features`` and detection masks
+        are in the undistorted image, whose camera is the sequence's K.  ``set_intrinsics`` and ``set_frame_size`` keep the
+        coefficients and rebuild the map.  Bad shapes, non-finite coefficients, bad indices or submitted frames still waiting
+        raise ValueError (the 12- and 14-coefficient models NotImplementedError) and change nothing.  The next step needs
+        prime().  Synchronous."""
+        seqs, d8 = _set_distortion(self.ctx, self.ctx.lib.b200vo_batch_set_distortion, self.h, self.batch, seqs, dist,
+                                   "b200vo_batch_set_distortion")
+        self.dist_coeffs[seqs] = d8
 
     def _frames(self, frames):
         """frames of a step: the slot-layout array, or a list of per-sequence 2-D images packed into it"""
@@ -354,11 +392,12 @@ class VOBatch:
     OK, IDLE, FEW_POINTS, PNP_FAILED, OVERFLOW, DETECT_LIMIT, NO_BOOTSTRAP = range(7)
 
     def __init__(self, batch, rows, cols, K, options, max_landmarks=4096, max_candidates=8192, max_frames=1024,
-                 frame_size=None, ctx: _lib.Context | None = None):
+                 frame_size=None, dist_coeffs=None, ctx: _lib.Context | None = None):
         self.ctx = ctx or _lib.default_context(0)
         self.batch, self.rows, self.cols = int(batch), int(rows), int(cols)
         self.frame_size = np.tile(np.int32([self.rows, self.cols]), (self.batch, 1))   # (batch, 2) rows, cols of every sequence
         self.has_mask = np.zeros(self.batch, bool)   # the sequences with a detection mask (set_detection_mask)
+        self.dist_coeffs = np.zeros((self.batch, 8))   # k1, k2, p1, p2, k3, k4, k5, k6 of every sequence (set_distortion)
         self._submitted = []
         self.L, self.Cn, self.P = int(max_landmarks), int(max_candidates), int(max_frames)
         self.options = options
@@ -373,6 +412,8 @@ class VOBatch:
             self.set_intrinsics(np.arange(self.batch), K_rows)
         if frame_size is not None:
             self.set_frame_size(np.arange(self.batch), frame_size)
+        if dist_coeffs is not None:
+            self.set_distortion(np.arange(self.batch), dist_coeffs)
         b = self.batch
         self._res = dict(status=self.pinned_empty((b,), np.int32), n_inliers=self.pinned_empty((b,), np.int32),
                          n_lm=self.pinned_empty((b,), np.int32), n_cand=self.pinned_empty((b,), np.int32),
@@ -438,6 +479,19 @@ class VOBatch:
                                    self.rows, self.cols, seqs, masks, "b200vo_loop_set_detection_mask")
         self.has_mask[seqs] = masks is not None
 
+    def set_distortion(self, seqs, dist):
+        """Give the distinct sequences ``seqs`` lens distortion: ``dist`` (len(seqs), n) with n = 4, 5 or 8 coefficients in cv2's
+        order (k1, k2, p1, p2[, k3[, k4, k5, k6]]), or None to clear it; an all-zero row clears it too.  Every frame the loop
+        takes for such a sequence (``step``, ``submit_frames``, ``load``, both frames of ``bootstrap``) is raw camera output,
+        undistorted on the device as ``cv2.undistort(frame, K, dist)`` does before anything reads it; states, ``read_state``,
+        poses and detection masks are in the undistorted image, whose camera is the sequence's K.  ``set_intrinsics`` and
+        ``set_frame_size`` keep the coefficients and rebuild the map.  The listed sequences become IDLE until ``load`` or
+        ``bootstrap``.  Bad shapes, non-finite coefficients, bad indices or submitted frames still waiting raise ValueError
+        (the 12- and 14-coefficient models NotImplementedError) and change nothing.  Synchronous."""
+        seqs, d8 = _set_distortion(self.ctx, self.ctx.lib.b200vo_loop_set_distortion, self.h, self.batch, seqs, dist,
+                                   "b200vo_loop_set_distortion")
+        self.dist_coeffs[seqs] = d8
+
     def load(self, seq: int, frame: np.ndarray, state: dict, K=None):
         """Set sequence ``seq`` to ``state`` (see the class docstring) with ``frame`` as its current frame; its status
         becomes OK.  ``K`` (3, 3): the sequence's camera from now on (``set_intrinsics`` first).  Out-of-range counts or
@@ -460,10 +514,17 @@ class VOBatch:
             K = np.asarray(K, np.float64)
             if K.shape != (3, 3) or not _pinhole(K):
                 raise ValueError("K must be a (3, 3) pinhole camera matrix (see set_intrinsics)")
+        K_first = K is not None and bool(self.dist_coeffs[int(seq)].any())
+        if K_first:
+            # the frame is undistorted with the sequence's K: it must be in place before the load, so the load's own
+            # refusals are checked here first to leave everything unchanged on bad input
+            if not (len(lm) <= self.L and len(keys) <= self.Cn and 1 <= len(poses) <= self.P) or (fp < 0).any() or (fp >= len(poses)).any():
+                raise ValueError("b200vo_loop_load: a count is out of range or a first_pose value outside [0, n_poses)")
+            self.set_intrinsics([seq], K[None])
         self._chk(self.ctx.lib.b200vo_loop_load(self.h, int(seq), _p(f, c_u8p), _p(lm, c_f32p), _p(kp, c_f32p), len(lm),
                                                 _p(keys, c_f32p), _p(fk, c_f32p), _p(fp, c_i32p), len(keys), _p(poses, c_f64p),
                                                 len(poses)), "b200vo_loop_load")
-        if K is not None:   # after the load, which is the call that can still refuse
+        if K is not None and not K_first:   # after the load, which is the call that can still refuse
             self.set_intrinsics([seq], K[None])
 
     def bootstrap(self, frames0, frames1, seqs=None, K=None) -> dict:
@@ -474,6 +535,8 @@ class VOBatch:
         arrays (len(seqs),): ``status`` (OK, NO_BOOTSTRAP or OVERFLOW), ``num_pts`` (the essential-matrix inlier count),
         ``n_lm`` and ``n_cand``.  A failing sequence keeps its state and is skipped by ``step`` until it is loaded or
         bootstrapped again.  ``K`` (len(seqs), 3, 3): the listed sequences' cameras from now on (``set_intrinsics`` first).
+        A sequence with distortion (``set_distortion``) runs on its undistorted frames: it ends up as ``load(s, frames1[k],
+        initial_state(K, options, *match_bootstrap_frames(undistort(frames0[k]), undistort(frames1[k]), ratio)))`` leaves it.
         Bad indices, frame shapes or K raise ValueError and change nothing.  Synchronous."""
         seqs = np.arange(self.batch, dtype=np.int32) if seqs is None else np.ascontiguousarray(seqs, np.int32).reshape(-1)
         if isinstance(frames0, (list, tuple)) or isinstance(frames1, (list, tuple)):

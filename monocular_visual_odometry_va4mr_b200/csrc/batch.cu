@@ -130,8 +130,47 @@ extern "C" int b200vo_batch_create(b200vo_ctx* ctx, int batch, const b200vo_batc
     rc = vo_reserve(ctx, B->ext_buf, (size_t)batch * sizeof(VoSeqExt));
     if (rc) { b200vo_batch_destroy(B); return rc; }
     B->mask_host.assign(batch, 0);   // no masks (and no mask buffer until the first one)
+    B->dist_host.assign((size_t)batch * 8, 0.0);   // no distortion (and no maps until the first one)
+    B->dist_on.assign(batch, 0);
     *out = B;
     return 0;
+}
+
+// the map of every listed sequence with distortion, from its K, coefficients and frame size (the work in flight has ended)
+static int batch_build_maps(b200vo_batch* B, int n_seq, const int32_t* seqs)
+{
+    b200vo_ctx* ctx = B->ctx;
+    const b200vo_batch_cfg& c = B->cfg;
+    std::vector<double> par;
+    std::vector<int32_t> im;
+    for (int k = 0; k < n_seq; ++k) {
+        const int s = seqs[k];
+        if (!B->dist_on[s]) continue;
+        const VoIntrinsics& r = B->intr_host[s];
+        const double* d = B->dist_host.data() + 8 * (size_t)s;
+        const double row[14] = {r.fx, r.fy, r.cx, r.cy, d[0], d[1], d[2], d[3], d[4], d[5], d[6], d[7],
+                                (double)B->ext_host[s].w[0], (double)B->ext_host[s].h[0]};
+        par.insert(par.end(), row, row + 14);
+        im.push_back(s);
+    }
+    if (im.empty()) return 0;
+    const size_t n = im.size(), b_par = vo_align(n * 14 * sizeof(double), 256), fb = (size_t)c.rows * c.cols;
+    VO_TRY(vo_reserve(ctx, B->dist_par, b_par + n * 4));
+    uint8_t* p = (uint8_t*)B->dist_par.p;
+    VO_CUDA(ctx, cudaMemcpyAsync(p, par.data(), par.size() * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+    VO_CUDA(ctx, cudaMemcpyAsync(p + b_par, im.data(), n * 4, cudaMemcpyHostToDevice, ctx->stream));
+    uint8_t* m = (uint8_t*)B->dist_buf.p + vo_align((size_t)B->batch, 256);
+    VO_TRY(vo_undistort_maps(ctx, (const double*)p, (const int*)(p + b_par), (int)n, c.rows, c.cols, (short2*)m,
+                             (uint16_t*)(m + (size_t)B->batch * fb * 4), fb, c.cols, ctx->stream));
+    VO_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    return 0;
+}
+
+static bool batch_any_dist(const b200vo_batch* B, int n_seq, const int32_t* seqs)
+{
+    bool any = false;
+    for (int k = 0; k < n_seq; ++k) any = any || (seqs[k] >= 0 && seqs[k] < B->batch && B->dist_on[seqs[k]]);
+    return any;
 }
 
 int batch_set_intrinsics(b200vo_batch* B, int n_seq, const int32_t* seqs, const double* K)
@@ -139,11 +178,17 @@ int batch_set_intrinsics(b200vo_batch* B, int n_seq, const int32_t* seqs, const 
     b200vo_ctx* ctx = B->ctx;
     std::vector<VoIntrinsics> rows = B->intr_host;
     VO_TRY(vo_intrinsics_set(ctx, B->batch, n_seq, seqs, K, VO_BOOT_EMAT_THR, rows.data()));
+    // a sequence with distortion undistorts its frames with K: the submitted sets were built with the old one
+    const bool remap = batch_any_dist(B, n_seq, seqs);
+    if (remap && B->q_count > 0)
+        return vo_set_err(ctx, B200VO_E_BADARG, "submitted frame sets are waiting: their pyramids were undistorted with the old K");
     VO_CUDA(ctx, cudaSetDevice(ctx->device));
     VO_CUDA(ctx, cudaStreamSynchronize(ctx->stream));   // no step in flight reads the rows (every stream of a step joins the ctx stream)
+    if (remap) VO_CUDA(ctx, cudaStreamSynchronize(B->pre_stream));
     VO_CUDA(ctx, cudaMemcpyAsync(B->intr_buf.p, rows.data(), rows.size() * sizeof(VoIntrinsics), cudaMemcpyHostToDevice, ctx->stream));
     VO_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     B->intr_host.swap(rows);
+    if (remap) VO_TRY(batch_build_maps(B, n_seq, seqs));
     return 0;
 }
 
@@ -187,6 +232,71 @@ int batch_set_frame_size(b200vo_batch* B, int n_seq, const int32_t* seqs, const 
     bool had_mask = false;
     for (int k = 0; k < n_seq; ++k) had_mask = had_mask || B->mask_host[seqs[k]];
     if (had_mask) VO_TRY(batch_set_detection_mask(B, n_seq, seqs, nullptr));
+    // a map covers its sequence's frame size: the listed sequences with distortion keep their coefficients, with new maps
+    VO_TRY(batch_build_maps(B, n_seq, seqs));
+    return 0;
+}
+
+int batch_set_distortion(b200vo_batch* B, int n_seq, const int32_t* seqs, const double* dist)
+{
+    b200vo_ctx* ctx = B->ctx;
+    const b200vo_batch_cfg& c = B->cfg;
+    if (n_seq < 1 || n_seq > B->batch) return vo_set_err(ctx, B200VO_E_BADARG, "n_seq = %d is outside [1, batch = %d]", n_seq, B->batch);
+    if (!seqs || !dist) return vo_set_err(ctx, B200VO_E_BADARG, "null array");
+    std::vector<char> seen(B->batch, 0);
+    for (int k = 0; k < n_seq; ++k) {
+        if (seqs[k] < 0 || seqs[k] >= B->batch)
+            return vo_set_err(ctx, B200VO_E_BADARG, "seqs[%d] = %d is outside [0, batch = %d)", k, seqs[k], B->batch);
+        if (seen[seqs[k]]++) return vo_set_err(ctx, B200VO_E_BADARG, "sequence %d is listed twice", seqs[k]);
+        if (!vo_dist_valid(dist + 8 * (size_t)k)) return vo_set_err(ctx, B200VO_E_BADARG, "sequence %d: non-finite distortion coefficient", seqs[k]);
+    }
+    if (B->q_count > 0) return vo_set_err(ctx, B200VO_E_BADARG, "submitted frame sets are waiting: their pyramids were built with the old maps");
+    std::vector<double> coef = B->dist_host;
+    std::vector<uint8_t> on = B->dist_on;
+    bool any_new = false;
+    for (int k = 0; k < n_seq; ++k) {
+        bool nz = false;
+        for (int i = 0; i < 8; ++i) nz = nz || dist[8 * (size_t)k + i] != 0.0;
+        for (int i = 0; i < 8; ++i) coef[8 * (size_t)seqs[k] + i] = nz ? dist[8 * (size_t)k + i] : 0.0;
+        on[seqs[k]] = nz ? 1 : 0;
+        any_new = any_new || nz;
+    }
+    const size_t fb = (size_t)c.rows * c.cols, b_on = vo_align((size_t)B->batch, 256);
+    VO_CUDA(ctx, cudaSetDevice(ctx->device));
+    VO_CUDA(ctx, cudaStreamSynchronize(ctx->stream));   // no step in flight reads the maps
+    VO_CUDA(ctx, cudaStreamSynchronize(B->pre_stream));
+    if (any_new) VO_TRY(vo_reserve(ctx, B->dist_buf, b_on + B->batch * fb * 6));
+    B->dist_host.swap(coef);
+    B->dist_on.swap(on);
+    if (B->dist_buf.p) {
+        VO_CUDA(ctx, cudaMemcpyAsync(B->dist_buf.p, B->dist_on.data(), B->dist_on.size(), cudaMemcpyHostToDevice, ctx->stream));
+        VO_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    }
+    return batch_build_maps(B, n_seq, seqs);
+}
+
+VoUndist batch_undist(const b200vo_batch* B, int b0, int n, const int32_t* list)
+{
+    VoUndist u;
+    bool any = false;
+    for (int k = 0; k < n; ++k) any = any || B->dist_on[list ? list[k] : b0 + k];
+    if (!any) return u;
+    const size_t fb = (size_t)B->cfg.rows * B->cfg.cols;
+    const uint8_t* d = (const uint8_t*)B->dist_buf.p;
+    const uint8_t* m = d + vo_align((size_t)B->batch, 256);
+    u.on = d + b0;
+    u.xy = (const short2*)m + b0 * fb;
+    u.fr = (const uint16_t*)(m + (size_t)B->batch * fb * 4) + b0 * fb;
+    u.stride = fb;
+    u.pitch = B->cfg.cols;
+    return u;
+}
+
+extern "C" int b200vo_batch_set_distortion(b200vo_batch* B, int n_seq, const int32_t* seqs, const double* dist)
+{
+    if (!B) return B200VO_E_BADARG;
+    VO_TRY(batch_set_distortion(B, n_seq, seqs, dist));
+    B->primed = false;   // the resident pyramids were built with the old maps
     return 0;
 }
 
@@ -311,7 +421,7 @@ extern "C" void b200vo_batch_destroy(b200vo_batch* B)
     kill_stream(B->pose_stream);
     for (auto& s : B->slabs) if (s.p) cudaFree(s.p);
     for (DevBuf* d : {&B->raw, &B->raw_pre, &B->pts_in, &B->outs, &B->work, &B->gftt_ws, &B->intr_buf, &B->ext_buf, &B->lists,
-                     &B->mask_buf})
+                     &B->mask_buf, &B->dist_buf, &B->dist_par})
         if (d->p) cudaFree(d->p);
     for (auto& e : B->q_ev) kill_event(e);
     for (auto& e : B->chunk_ev) kill_event(e);
@@ -339,7 +449,8 @@ static int batch_upload_frames(b200vo_batch* B, const uint8_t* frames, int slab_
     }
     VO_CUDA(ctx, cudaMemcpyAsync(B->raw.p, src, total, cudaMemcpyHostToDevice, ctx->stream));
     VO_TRY(vo_build_pyramids(ctx, (const uint8_t*)B->raw.p, fb, B->cfg.rows, B->cfg.cols, B->geom,
-                             (uint8_t*)B->slabs[slab_set].p, B->geom.slab_bytes, B->batch, ctx->stream, batch_ext_dev(B, 0), batch_ext_host(B, 0)));
+                             (uint8_t*)B->slabs[slab_set].p, B->geom.slab_bytes, B->batch, ctx->stream, batch_ext_dev(B, 0), batch_ext_host(B, 0),
+                             0, nullptr, nullptr, 0, batch_undist(B, 0, B->batch)));
     return 0;
 }
 
@@ -432,11 +543,11 @@ int batch_issue_prefetch(b200vo_batch* B, cudaEvent_t after, bool wait_step_end)
         if (ql.empty())
             VO_TRY(vo_build_pyramids(ctx, raw, fb, B->cfg.rows, B->cfg.cols, B->geom,
                                      (uint8_t*)B->slabs[B->q_set[slot]].p, B->geom.slab_bytes, B->batch, B->pre_stream, batch_ext_dev(B, 0),
-                                     batch_ext_host(B, 0)));
+                                     batch_ext_host(B, 0), 0, nullptr, nullptr, 0, batch_undist(B, 0, B->batch)));
         else
             VO_TRY(vo_build_pyramids(ctx, raw, fb, B->cfg.rows, B->cfg.cols, B->geom, (uint8_t*)B->slabs[B->q_set[slot]].p,
                                      B->geom.slab_bytes, (int)ql.size(), B->pre_stream, batch_ext_dev(B, 0), batch_ext_host(B, 0), 0,
-                                     batch_list_row(B, slot), ql.data(), B->batch));
+                                     batch_list_row(B, slot), ql.data(), B->batch, batch_undist(B, 0, (int)ql.size(), ql.data())));
         VO_CUDA(ctx, cudaEventRecord(B->q_ev[slot], B->pre_stream));
         B->q_src[slot] = nullptr;
     }
@@ -476,10 +587,12 @@ static int batch_track(b200vo_batch* B, cudaStream_t stream, int b0, int nb, con
         if (whole) prof_mark(B, 0, stream);
         if (frames_dev && B->step_list)   // the listed images into their sequences' slabs (b0 == 0, nb == batch)
             VO_TRY(vo_build_pyramids(ctx, frames_dev, fb, c.rows, c.cols, B->geom, (uint8_t*)B->slabs[nxt].p, sb, B->step_n, stream,
-                                     batch_ext_dev(B, 0), batch_ext_host(B, 0), 0, B->step_list, B->step_list_host, B->batch));
+                                     batch_ext_dev(B, 0), batch_ext_host(B, 0), 0, B->step_list, B->step_list_host, B->batch,
+                                     batch_undist(B, 0, B->step_n, B->step_list_host)));
         else if (frames_dev)
             VO_TRY(vo_build_pyramids(ctx, frames_dev + (size_t)b0 * fb, fb, c.rows, c.cols, B->geom,
-                                     (uint8_t*)B->slabs[nxt].p + (size_t)b0 * sb, sb, nb, stream, batch_ext_dev(B, b0), batch_ext_host(B, b0)));
+                                     (uint8_t*)B->slabs[nxt].p + (size_t)b0 * sb, sb, nb, stream, batch_ext_dev(B, b0), batch_ext_host(B, b0),
+                                     0, nullptr, nullptr, 0, batch_undist(B, b0, nb)));
         if (whole) { prof_mark(B, 1, stream); B->prof_row_open = B->profile && B->prof_n < B200VO_PROF_RING; }
     }
     KltPointSet sets[2] = {{L, n_lm + b0, lm_pts + (size_t)b0 * L * 2, lm_next + (size_t)b0 * L * 2, lm_status + (size_t)b0 * L, nullptr},

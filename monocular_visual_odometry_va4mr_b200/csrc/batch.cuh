@@ -66,6 +66,13 @@ struct b200vo_batch {
     // in the slot layout, allocated with the first mask.  mask_host mirrors the flags; no flag set: the detectors get no mask.
     DevBuf mask_buf;
     std::vector<uint8_t> mask_host;
+    // the lens distortion of every sequence (b200vo_batch_set_distortion): [batch] "has distortion" bytes, then [batch]
+    // int16 source-pixel maps and [batch] uint16 fraction maps in the slot layout (VoUndist), allocated with the first
+    // distortion.  dist_host: the coefficients, [batch][8]; dist_on mirrors the flags; no flag set: pyramids as without.
+    DevBuf dist_buf;
+    DevBuf dist_par;                // the parameter rows of the last map build
+    std::vector<double> dist_host;
+    std::vector<uint8_t> dist_on;
     // host-input path: frames arrive chunk by chunk on a copy stream while earlier chunks are tracked
     cudaStream_t chunk_stream[B200VO_BATCH_STREAMS] = {};  // chunk k: H2D -> pyramid -> KLT on stream k % STREAMS
     cudaEvent_t chunk_ev[B200VO_BATCH_CHUNKS] = {};
@@ -110,6 +117,12 @@ int batch_set_frame_size(b200vo_batch* B, int n_seq, const int32_t* seqs, const 
 int batch_set_detection_mask(b200vo_batch* B, int n_seq, const int32_t* seqs, const uint8_t* masks);
 // the masks of the detectors: indexed by sequence, none while no sequence has one
 VoMask batch_mask(const b200vo_batch* B);
+// Validates the n_seq distinct indices and their coefficients (dist: [n_seq][8] k1, k2, p1, p2, k3, k4, k5, k6; an
+// all-zero row clears a sequence's distortion) and, only when all are valid and no submitted frame set waits, waits for
+// the work in flight and builds the listed sequences' maps.  Synchronous.
+int batch_set_distortion(b200vo_batch* B, int n_seq, const int32_t* seqs, const double* dist);
+// the maps of sequences b0 .. b0 + n - 1, or of the n sequences list[k] (b0 == 0); none while none of them has distortion
+VoUndist batch_undist(const b200vo_batch* B, int b0, int n, const int32_t* list = nullptr);
 // the device rows of sequences [b0, ...) and their host copy, or nullptr for both while every sequence has the slot size
 inline const VoSeqExt* batch_ext_dev(const b200vo_batch* B, int b0) { return B->ext ? B->ext + b0 : nullptr; }
 inline const VoSeqExt* batch_ext_host(const b200vo_batch* B, int b0) { return B->ext ? B->ext_host.data() + b0 : nullptr; }

@@ -142,6 +142,7 @@ extern "C" void b200vo_destroy(b200vo_ctx* ctx)
     if (ctx->d_rng.p) cudaFree(ctx->d_rng.p);
     if (ctx->d_intr.p) cudaFree(ctx->d_intr.p);
     if (ctx->d_mask.p) cudaFree(ctx->d_mask.p);
+    if (ctx->d_undist.p) cudaFree(ctx->d_undist.p);
     if (ctx->d_sift.p) cudaFree(ctx->d_sift.p);
     for (DevBuf* b : {&ctx->d_sift_out[0], &ctx->d_sift_out[1], &ctx->d_sift_sort}) if (b->p) cudaFree(b->p);
     if (ctx->d_klt_queue.p) cudaFree(ctx->d_klt_queue.p);

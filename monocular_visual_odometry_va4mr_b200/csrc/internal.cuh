@@ -50,6 +50,34 @@ struct VoMask {
     int pitch = 0;
 };
 
+// Lens distortion (cv2.undistort with newCameraMatrix = K): image im's fixed-point map in cv2's CV_16SC2 + CV_16UC1
+// layout, entry (x, y) at im * stride + y * pitch + x: xy = the source pixel (saturated to int16), fr = (v & 31) * 32 +
+// (u & 31) in 1/32 px.  on[im] == 0: image im has no distortion (copied as is); on == nullptr: every image has one.
+// xy == nullptr: no image of the launch has distortion, and the pyramid builder runs exactly as without this argument.
+struct VoUndist {
+    const short2* xy = nullptr;
+    const uint16_t* fr = nullptr;
+    const uint8_t* on = nullptr;
+    size_t stride = 0;
+    int pitch = 0;
+};
+
+// Pixel (x, y) of the undistorted w x h image whose map is xy / fr, rows `pitch` entries apart (cv2.remap, INTER_LINEAR, BORDER_CONSTANT 0):
+// fixed-point bilinear with 1/32 px weights, each tap outside the raw image (rows `row` bytes apart) contributing 0
+__device__ __forceinline__ uint32_t vo_undist_px(const uint8_t* __restrict__ src, size_t row, int w, int h, const short2* xy,
+                                                 const uint16_t* fr, int pitch, int x, int y)
+{
+    const int i = y * pitch + x;
+    const short2 s = xy[i];
+    const int f = fr[i], ax = f & 31, ay = f >> 5;
+    auto tap = [&](int yy, int xx) -> int {
+        return ((unsigned)xx < (unsigned)w && (unsigned)yy < (unsigned)h) ? (int)__ldg(src + (size_t)yy * row + xx) : 0;
+    };
+    const int sum = tap(s.y, s.x) * (32 - ax) * (32 - ay) + tap(s.y, s.x + 1) * ax * (32 - ay) +
+                    tap(s.y + 1, s.x) * (32 - ax) * ay + tap(s.y + 1, s.x + 1) * ax * ay;
+    return (uint32_t)((32 * sum + (1 << 14)) >> 15);
+}
+
 struct KltParams {
     int win_w, win_h;
     int max_count;
@@ -115,6 +143,7 @@ struct b200vo_ctx {
     int n_rng = 0;
     DevBuf d_intr;           // the one-row intrinsics array of the one-call entry points (vo_intrinsics_one)
     DevBuf d_mask;           // the detection mask of the masked one-call entry points
+    DevBuf d_undist;         // the map of b200vo_undistort
     // tensor-map encode entry point (driver API, fetched lazily)
     void* encode_tiled = nullptr;
 };
@@ -182,10 +211,24 @@ void vo_seq_ext(int rows, int cols, int win_w, int win_h, int max_level, VoSeqEx
 // slot geometry g; every level of a sequence is built at its own size, levels beyond its own count are not built.
 // d_list / h_list (both or neither): raw image k goes to slab list[k] of the n_slab slabs at d_slab, with the extents
 // ext[list[k]] (the tables then cover all n_slab slabs); the other slabs are not touched.
+// ud: the images' distortion maps, indexed like the extents (by slab); level 0 is then the undistorted image.
 int vo_build_pyramids(b200vo_ctx* ctx, const uint8_t* d_raw, size_t raw_stride, int rows, int cols,
                       const PyrGeom& g, uint8_t* d_slab, size_t slab_stride, int batch, cudaStream_t stream,
                       const VoSeqExt* d_ext = nullptr, const VoSeqExt* h_ext = nullptr, size_t raw_row = 0,
-                      const int* d_list = nullptr, const int* h_list = nullptr, int n_slab = 0);
+                      const int* d_list = nullptr, const int* h_list = nullptr, int n_slab = 0, const VoUndist& ud = VoUndist{});
+
+// ---- undistort.cu ----
+// The 8 coefficients k1, k2, p1, p2, k3, k4, k5, k6 are finite (what *_set_distortion and b200vo_undistort accept)
+bool vo_dist_valid(const double d[8]);
+// map of image im = 0 .. n-1 (cv2.initUndistortRectifyMap(K, d, None, K, (cols[im], rows[im]), CV_16SC2)) into
+// xy / fr + im_of[im] * stride, rows `pitch` entries apart.  par: [n][14] doubles fx, fy, cx, cy, k1 .. k6, cols, rows.
+int vo_undistort_maps(b200vo_ctx* ctx, const double* d_par, const int* d_im_of, int n, int max_rows, int max_cols, short2* xy,
+                      uint16_t* fr, size_t stride, int pitch, cudaStream_t stream);
+// raw frames z = 0 .. n-1 (rows of `row` bytes, `stride` apart) -> undistorted frames at dst (same layout).  Frame z is
+// image seq_of[z >> seq_shift] of ud (seq_of == nullptr: image z) at that image's size: ext[image] (nullptr: rows x cols).
+// An image without distortion is copied.
+int vo_undistort_frames(b200vo_ctx* ctx, const uint8_t* src, uint8_t* dst, size_t stride, size_t row, int n, int rows, int cols,
+                        const VoUndist& ud, const int* seq_of, int seq_shift, const VoSeqExt* ext, cudaStream_t stream);
 
 // ---- gftt.cu: detection on device-resident bordered level-0 images, one per batch entry ----
 #define VO_GFTT_SMALL 4          // ints per image in the result block: max bits | n candidates | n corners | spare

@@ -555,7 +555,8 @@ extern "C" int b200vo_loop_load(b200vo_loop* lp, int seq, const uint8_t* frame, 
     VO_TRY(vo_reserve(ctx, B->raw, fb));
     VO_CUDA(ctx, cudaMemcpy2DAsync(B->raw.p, (size_t)cols, frame, (size_t)cs, (size_t)cs, (size_t)rs, cudaMemcpyHostToDevice, st));
     VO_TRY(vo_build_pyramids(ctx, (const uint8_t*)B->raw.p, fb, rows, cols, B->geom,
-                             (uint8_t*)B->slabs[B->cur].p + (size_t)seq * sb, sb, 1, st, batch_ext_dev(B, seq), batch_ext_host(B, seq)));
+                             (uint8_t*)B->slabs[B->cur].p + (size_t)seq * sb, sb, 1, st, batch_ext_dev(B, seq), batch_ext_host(B, seq),
+                             0, nullptr, nullptr, 0, batch_undist(B, seq, 1)));
     const size_t lo = (size_t)seq * d.L, co = (size_t)seq * d.C;
     if (n_lm > 0) {
         VO_CUDA(ctx, cudaMemcpyAsync(d.lm + 3 * lo, lm, (size_t)n_lm * 12, cudaMemcpyHostToDevice, st));
@@ -579,12 +580,10 @@ extern "C" int b200vo_loop_set_intrinsics(b200vo_loop* lp, int n_seq, const int3
     return lp ? batch_set_intrinsics(lp->B, n_seq, seqs, K) : B200VO_E_BADARG;
 }
 
-extern "C" int b200vo_loop_set_frame_size(b200vo_loop* lp, int n_seq, const int32_t* seqs, const int32_t* rows, const int32_t* cols)
+// the listed sequences' pyramids no longer match their frames: IDLE (state arrays kept) until loaded or bootstrapped
+static int loop_idle(b200vo_loop* lp, int n_seq, const int32_t* seqs)
 {
-    if (!lp) return B200VO_E_BADARG;
     b200vo_ctx* ctx = lp->ctx;
-    VO_TRY(batch_set_frame_size(lp->B, n_seq, seqs, rows, cols));
-    // the listed sequences' pyramids no longer match their frames: IDLE (state arrays kept) until loaded or bootstrapped
     const int idle = B200VO_LOOP_IDLE, zero = 0;
     const LoopDev& d = lp->d;
     for (int k = 0; k < n_seq; ++k) {
@@ -594,6 +593,20 @@ extern "C" int b200vo_loop_set_frame_size(b200vo_loop* lp, int n_seq, const int3
     }
     VO_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     return 0;
+}
+
+extern "C" int b200vo_loop_set_frame_size(b200vo_loop* lp, int n_seq, const int32_t* seqs, const int32_t* rows, const int32_t* cols)
+{
+    if (!lp) return B200VO_E_BADARG;
+    VO_TRY(batch_set_frame_size(lp->B, n_seq, seqs, rows, cols));
+    return loop_idle(lp, n_seq, seqs);
+}
+
+extern "C" int b200vo_loop_set_distortion(b200vo_loop* lp, int n_seq, const int32_t* seqs, const double* dist)
+{
+    if (!lp) return B200VO_E_BADARG;
+    VO_TRY(batch_set_distortion(lp->B, n_seq, seqs, dist));
+    return loop_idle(lp, n_seq, seqs);
 }
 
 extern "C" int b200vo_loop_set_detection_mask(b200vo_loop* lp, int n_seq, const int32_t* seqs, const uint8_t* masks)
@@ -786,10 +799,15 @@ extern "C" int b200vo_loop_bootstrap(b200vo_loop* lp, int n_seq, const int32_t* 
     cudaStream_t st = ctx->stream;
     // the two frames of sequence j of the run are frames 2j and 2j + 1 of the SIFT batch (slot layout)
     const size_t b_raw = vo_align(ns * 2 * fb, 256), b_cnt = vo_align(ns * 8, 256), b_moff = vo_align(ns * 16, 256);
-    VO_TRY(vo_reserve(ctx, lp->boot_in, b_raw + 2 * b_cnt + b_moff));
+    // sequences with distortion: the raw frames land in a staging area and are undistorted into `raw`, which then holds
+    // every frame as SIFT and the second frame's pyramid read it (the pyramid build does not undistort again)
+    const VoUndist ud = batch_undist(B, 0, n_seq, seqs);
+    const size_t b_seq = vo_align(ns * 4, 256), b_stage = ud.xy ? b_raw + b_seq : 0;
+    VO_TRY(vo_reserve(ctx, lp->boot_in, b_raw + 2 * b_cnt + b_moff + b_stage));
     uint8_t* raw = (uint8_t*)lp->boot_in.p;
     int* d_nkp = (int*)(raw + b_raw);
     int* d_row = (int*)(raw + b_raw + b_cnt);
+    uint8_t* in = ud.xy ? raw + b_raw + 2 * b_cnt + b_moff : raw;   // where the raw frames land
     // both SIFT frames of a sequence with a detection mask use it: the offsets of the run's frames in the mask slab
     const VoMask mk = batch_mask(B);
     long long* d_moff = nullptr;
@@ -800,13 +818,18 @@ extern "C" int b200vo_loop_bootstrap(b200vo_loop* lp, int n_seq, const int32_t* 
         VO_CUDA(ctx, cudaMemcpyAsync(d_moff, moff.data(), ns * 16, cudaMemcpyHostToDevice, st));
     }
     if (in_order) {
-        VO_CUDA(ctx, cudaMemcpy2DAsync(raw, 2 * fb, frames0, fb, fb, ns, cudaMemcpyHostToDevice, st));
-        VO_CUDA(ctx, cudaMemcpy2DAsync(raw + fb, 2 * fb, frames1, fb, fb, ns, cudaMemcpyHostToDevice, st));
+        VO_CUDA(ctx, cudaMemcpy2DAsync(in, 2 * fb, frames0, fb, fb, ns, cudaMemcpyHostToDevice, st));
+        VO_CUDA(ctx, cudaMemcpy2DAsync(in + fb, 2 * fb, frames1, fb, fb, ns, cudaMemcpyHostToDevice, st));
     } else {
         for (int j = 0; j < n_seq; ++j) {
-            VO_CUDA(ctx, cudaMemcpyAsync(raw + 2 * j * fb, frames0 + (size_t)perm[j] * fb, fb, cudaMemcpyHostToDevice, st));
-            VO_CUDA(ctx, cudaMemcpyAsync(raw + (2 * j + 1) * fb, frames1 + (size_t)perm[j] * fb, fb, cudaMemcpyHostToDevice, st));
+            VO_CUDA(ctx, cudaMemcpyAsync(in + 2 * j * fb, frames0 + (size_t)perm[j] * fb, fb, cudaMemcpyHostToDevice, st));
+            VO_CUDA(ctx, cudaMemcpyAsync(in + (2 * j + 1) * fb, frames1 + (size_t)perm[j] * fb, fb, cudaMemcpyHostToDevice, st));
         }
+    }
+    if (ud.xy) {   // frames 2j and 2j + 1 are sequence seqs[j]'s (run order)
+        int* d_seq = (int*)(in + b_raw);
+        VO_CUDA(ctx, cudaMemcpyAsync(d_seq, seqs, ns * 4, cudaMemcpyHostToDevice, st));
+        VO_TRY(vo_undistort_frames(ctx, in, raw, fb, (size_t)cols, 2 * n_seq, rows, cols, ud, d_seq, 1, batch_ext_dev(B, 0), st));
     }
     // SIFT per size group, each group's keypoint and descriptor rows after the previous group's
     int n_rows = 0;

@@ -70,11 +70,14 @@ __device__ __forceinline__ int reflect101(int p, int len)
 }
 
 // raw image (rows of raw_row bytes) -> bordered level 0.  One thread = one 16-byte store of the bordered row.
-// ext: the sequence's own width and height (the grid covers the slot's); list: raw image z goes to slab list[z]
+// ext: the sequence's own width and height (the grid covers the slot's); list: raw image z goes to slab list[z].
+// UD: level 0 of a sequence with distortion is its undistorted image, gathered through its map; a ring pixel is the
+// REFLECT_101 of the undistorted image, so it takes the map entry of the interior pixel it mirrors.
+template <bool UD>
 __global__ void __launch_bounds__(256)
 pad_level0_kernel(const uint8_t* __restrict__ raw, size_t raw_stride, size_t raw_row, int w, int h,
                   uint8_t* __restrict__ slab, size_t slab_stride, size_t off0, int pitch, const VoSeqExt* __restrict__ ext,
-                  const int* __restrict__ list)
+                  const int* __restrict__ list, VoUndist ud)
 {
     const int seq = list ? list[blockIdx.z] : blockIdx.z;
     if (ext) { w = ext[seq].w[0]; h = ext[seq].h[0]; }
@@ -84,6 +87,24 @@ pad_level0_kernel(const uint8_t* __restrict__ raw, size_t raw_stride, size_t raw
     const int gy = blockIdx.y * blockDim.y + threadIdx.y - VO_BORDER;
     if (gx >= w + VO_BORDER || gy >= h + VO_BORDER) return;
     const int sy = reflect101(gy, h);
+    if (UD && (!ud.on || ud.on[seq])) {
+        const short2* xy = ud.xy + seq * ud.stride;
+        const uint16_t* fr = ud.fr + seq * ud.stride;
+        uint32_t v[4];
+#pragma unroll
+        for (int k = 0; k < 4; ++k) {
+            uint32_t acc = 0;
+#pragma unroll
+            for (int b = 0; b < 4; ++b) {
+                const int x = gx + 4 * k + b;
+                const uint32_t px = (x < w + VO_BORDER) ? vo_undist_px(src, raw_row, w, h, xy, fr, ud.pitch, reflect101(x, w), sy) : 0u;
+                acc |= px << (8 * b);
+            }
+            v[k] = acc;
+        }
+        *reinterpret_cast<uint4*>(dst + (long long)gy * pitch + gx) = make_uint4(v[0], v[1], v[2], v[3]);
+        return;
+    }
     const uint8_t* srow = src + (size_t)sy * raw_row;
     uint32_t v[4];
     if (gx >= 0 && gx + 15 < w) {
@@ -327,7 +348,8 @@ static int pyr_src_map(b200vo_ctx* ctx, CUtensorMap* map, uint8_t* d_slab, size_
 
 int vo_build_pyramids(b200vo_ctx* ctx, const uint8_t* d_raw, size_t raw_stride, int rows, int cols,
                       const PyrGeom& g, uint8_t* d_slab, size_t slab_stride, int batch, cudaStream_t stream,
-                      const VoSeqExt* d_ext, const VoSeqExt* h_ext, size_t raw_row, const int* d_list, const int* h_list, int n_slab)
+                      const VoSeqExt* d_ext, const VoSeqExt* h_ext, size_t raw_row, const int* d_list, const int* h_list, int n_slab,
+                      const VoUndist& ud)
 {
     if (!raw_row) raw_row = (size_t)cols;
     // the slabs the tensor maps span: every slab of the set when the images go to listed slabs
@@ -336,8 +358,12 @@ int vo_build_pyramids(b200vo_ctx* ctx, const uint8_t* d_raw, size_t raw_stride, 
         dim3 block(32, 8);
         int gxn = (cols + 2 * VO_BORDER + 15) / 16;
         dim3 grid((gxn + block.x - 1) / block.x, (rows + 2 * VO_BORDER + block.y - 1) / block.y, batch);
-        pad_level0_kernel<<<grid, block, 0, stream>>>(d_raw, raw_stride, raw_row, cols, rows, d_slab, slab_stride,
-                                                       g.off[0], g.pitch[0], d_ext, d_list);
+        if (ud.xy)   // the gathering instance only when some image of the launch has distortion
+            pad_level0_kernel<true><<<grid, block, 0, stream>>>(d_raw, raw_stride, raw_row, cols, rows, d_slab, slab_stride,
+                                                                g.off[0], g.pitch[0], d_ext, d_list, ud);
+        else
+            pad_level0_kernel<false><<<grid, block, 0, stream>>>(d_raw, raw_stride, raw_row, cols, rows, d_slab, slab_stride,
+                                                                 g.off[0], g.pitch[0], d_ext, d_list, ud);
         ctx->launches++;
     }
     if (g.levels > 1) {

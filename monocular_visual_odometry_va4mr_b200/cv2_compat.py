@@ -406,6 +406,43 @@ def recoverPose(E, points1, points2, cameraMatrix=None, R=None, t=None, mask=Non
 
 
 # --------------------------------------------------------------------------------------
+# cv2.undistort  (raw frames of cameras with lens distortion)
+# --------------------------------------------------------------------------------------
+def undistort(src, cameraMatrix, distCoeffs, dst=None, newCameraMatrix=None):
+    """cv2.undistort(src, cameraMatrix, distCoeffs) -> uint8 image of src's shape, byte for byte what cv2 computes.  src: 2-D
+    uint8.  distCoeffs: 4, 5 or 8 coefficients (k1, k2, p1, p2[, k3[, k4, k5, k6]]) or None (a copy).  newCameraMatrix
+    other than None or cameraMatrix, multi-channel images, the 12- and 14-coefficient models and a cameraMatrix with skew
+    raise ``NotImplementedError``; a bad cameraMatrix or non-finite coefficients raise ``error``."""
+    if isinstance(src, np.ndarray) and src.ndim == 3:
+        raise NotImplementedError("b200vo undistort: single-channel images only")
+    src, step = _image_arg(src, "src")
+    K = np.asarray(cameraMatrix, np.float64)
+    if K.shape != (3, 3):
+        raise error("b200vo undistort: (-215:Assertion failed) cameraMatrix is 3x3")
+    K = np.ascontiguousarray(K)
+    if newCameraMatrix is not None and not np.array_equal(np.asarray(newCameraMatrix, np.float64), K):
+        raise NotImplementedError("b200vo undistort: newCameraMatrix must be None or cameraMatrix")
+    if K[0, 1] != 0 or K[1, 0] != 0 or K[2, 0] != 0 or K[2, 1] != 0 or K[2, 2] != 1:
+        raise NotImplementedError("b200vo undistort: only pinhole camera matrices (no skew, last row 0 0 1)")
+    d = np.zeros(4) if distCoeffs is None else np.asarray(distCoeffs, np.float64).reshape(-1)
+    if d.size in (12, 14):
+        raise NotImplementedError("b200vo undistort: the thin-prism (12) and tilted (14) models are not supported")
+    if d.size not in (4, 5, 8):
+        raise error("b200vo undistort: (-215:Assertion failed) distCoeffs has 4, 5, 8, 12 or 14 elements")
+    d = np.ascontiguousarray(d)
+    out = np.empty(src.shape, np.uint8)
+    ctx = _ctx()
+    rc = ctx.lib.b200vo_undistort(ctx.h, _p(src, c_u8p), src.shape[0], src.shape[1], step, _p(K, c_f64p), _p(d, c_f64p), d.size,
+                                  _p(out, c_u8p))
+    if rc != 0:
+        _raise(ctx, rc, "undistort")
+    if dst is not None:
+        dst[...] = out
+        return dst
+    return out
+
+
+# --------------------------------------------------------------------------------------
 # cv2.solvePnPRansac  (reference :343)
 # --------------------------------------------------------------------------------------
 def solvePnPRansac(objectPoints, imagePoints, cameraMatrix, distCoeffs, rvec=None, tvec=None,
