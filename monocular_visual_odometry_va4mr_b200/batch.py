@@ -38,80 +38,6 @@ def _pinhole(K) -> bool:
                 and K[2, 1] == 0 and K[2, 2] == 1)
 
 
-def _set_intrinsics(ctx, fn, h, batch, seqs, K, what):
-    """Shared body of SequenceBatch / VOBatch.set_intrinsics."""
-    seqs = np.ascontiguousarray(seqs, np.int32).reshape(-1)
-    K = np.ascontiguousarray(K, np.float64)
-    if K.shape != (len(seqs), 3, 3):
-        raise ValueError(f"K must be (len(seqs) = {len(seqs)}, 3, 3), got {K.shape}")
-    rc = fn(h, len(seqs), _p(seqs, c_i32p), _p(K, c_f64p))
-    if rc == -1:
-        raise ValueError(f"{what}: {ctx.last_error()}")
-    if rc != 0:
-        raise _lib.B200VOError(f"{what} failed ({rc}): {ctx.last_error()}")
-
-
-def _set_frame_size(ctx, fn, h, seqs, sizes, what):
-    """Shared body of SequenceBatch / VOBatch.set_frame_size.  -> (seqs, sizes) as the call took them."""
-    seqs = np.ascontiguousarray(seqs, np.int32).reshape(-1)
-    sizes = np.asarray(sizes)
-    if sizes.shape != (len(seqs), 2) or not np.issubdtype(sizes.dtype, np.integer):
-        raise ValueError(f"sizes must be integer (len(seqs) = {len(seqs)}, 2) (rows, cols), got {sizes.dtype} {sizes.shape}")
-    rows = np.ascontiguousarray(sizes[:, 0], np.int32)
-    cols = np.ascontiguousarray(sizes[:, 1], np.int32)
-    rc = fn(h, len(seqs), _p(seqs, c_i32p), _p(rows, c_i32p), _p(cols, c_i32p))
-    if rc == -1:
-        raise ValueError(f"{what}: {ctx.last_error()}")
-    if rc != 0:
-        raise _lib.B200VOError(f"{what} failed ({rc}): {ctx.last_error()}")
-    return seqs, np.stack([rows, cols], 1)
-
-
-def _set_detection_mask(ctx, fn, h, batch, frame_size, rows, cols, seqs, masks, what):
-    """Shared body of SequenceBatch / VOBatch.set_detection_mask.  -> the int32 seqs the call took."""
-    seqs = np.asarray(seqs)
-    if seqs.ndim != 1 or not 1 <= seqs.size <= batch or not np.issubdtype(seqs.dtype, np.integer):
-        raise ValueError(f"seqs must be 1 to batch = {batch} integer sequence indices, got {seqs.dtype} {seqs.shape}")
-    if ((seqs < 0) | (seqs >= batch)).any():
-        raise ValueError(f"seqs must lie in [0, batch = {batch})")
-    seqs = np.ascontiguousarray(seqs, np.int32)
-    if masks is not None:
-        if isinstance(masks, (list, tuple)):
-            masks = _pack_frames(list(masks), frame_size[seqs], rows, cols)
-        masks = np.asarray(masks)
-        if masks.dtype != np.uint8 or masks.shape != (len(seqs), rows, cols):
-            raise ValueError(f"masks must be ({len(seqs)}, {rows}, {cols}) uint8 or a list of {len(seqs)} masks, got {masks.dtype} {masks.shape}")
-        masks = np.ascontiguousarray(masks)
-    rc = fn(h, len(seqs), _p(seqs, c_i32p), None if masks is None else _p(masks, c_u8p))
-    if rc == -1:
-        raise ValueError(f"{what}: {ctx.last_error()}")
-    if rc != 0:
-        raise _lib.B200VOError(f"{what} failed ({rc}): {ctx.last_error()}")
-    return seqs
-
-
-def _set_distortion(ctx, fn, h, batch, seqs, dist, what):
-    """Shared body of SequenceBatch / VOBatch.set_distortion.  -> (seqs, dist (len(seqs), 8)) as the call took them."""
-    seqs = np.asarray(seqs)
-    if seqs.ndim != 1 or not 1 <= seqs.size <= batch or not np.issubdtype(seqs.dtype, np.integer):
-        raise ValueError(f"seqs must be 1 to batch = {batch} integer sequence indices, got {seqs.dtype} {seqs.shape}")
-    seqs = np.ascontiguousarray(seqs, np.int32)
-    d8 = np.zeros((len(seqs), 8), np.float64)
-    if dist is not None:
-        d = np.asarray(dist)
-        if d.ndim == 2 and d.shape[0] == len(seqs) and d.shape[1] in (12, 14):
-            raise NotImplementedError("the thin-prism (12) and tilted (14) distortion models are not supported")
-        if d.ndim != 2 or d.shape[0] != len(seqs) or d.shape[1] not in (4, 5, 8) or not np.issubdtype(d.dtype, np.number):
-            raise ValueError(f"dist must be (len(seqs) = {len(seqs)}, 4 | 5 | 8) coefficients or None, got {d.dtype} {d.shape}")
-        d8[:, :d.shape[1]] = d
-    rc = fn(h, len(seqs), _p(seqs, c_i32p), _p(d8, c_f64p))
-    if rc == -1:
-        raise ValueError(f"{what}: {ctx.last_error()}")
-    if rc != 0:
-        raise _lib.B200VOError(f"{what} failed ({rc}): {ctx.last_error()}")
-    return seqs, d8
-
-
 def _pack_frames(frames, sizes, rows, cols, out=None):
     """A list of per-sequence 2-D uint8 images, each of its sequence's (rows_s, cols_s), packed into the slot layout
     (len, rows, cols); the bytes outside each image are zero.  An array is returned as it is."""
@@ -159,17 +85,160 @@ class _PinnedBlock:
             pass
 
 
-class SequenceBatch:
-    def __init__(self, batch, rows, cols, K, win=(15, 15), max_level=5, criteria=(3, 50, 0.01),
-                 min_eig_thr=1e-4, pnp_iters=500, pnp_reproj_err=8.0, pnp_conf=0.99,
-                 max_landmarks=1024, max_candidates=1024, frame_size=None, dist_coeffs=None, ctx: _lib.Context | None = None):
+class _Batch:
+    """What SequenceBatch and VOBatch share: the C object of the functions ``<prefix>*`` (``b200vo_batch_`` or
+    ``b200vo_loop_``) and its lifetime, page-locked arrays, and the settings every sequence has of its own -- camera
+    matrix, frame size, detection mask and lens distortion -- with their host mirrors ``frame_size``, ``has_mask`` and
+    ``dist_coeffs``."""
+
+    def __init__(self, prefix, batch, rows, cols, ctx):
+        self._prefix = prefix
         self.ctx = ctx or _lib.default_context(0)
         self.batch, self.rows, self.cols = int(batch), int(rows), int(cols)
-        self.L, self.Cn = int(max_landmarks), int(max_candidates)
         self.frame_size = np.tile(np.int32([self.rows, self.cols]), (self.batch, 1))   # (batch, 2) rows, cols of every sequence
         self.has_mask = np.zeros(self.batch, bool)   # the sequences with a detection mask (set_detection_mask)
         self.dist_coeffs = np.zeros((self.batch, 8))   # k1, k2, p1, p2, k3, k4, k5, k6 of every sequence (set_distortion)
         self._submitted = []   # page-locked slot-layout copies of submitted frame lists, alive until their step
+
+    def _create(self, cfg, K_rows, frame_size, dist_coeffs):
+        """Creates the C object from ``cfg``, then applies the constructor's per-sequence K rows, frame sizes and distortion."""
+        self.cfg = cfg
+        h = C.c_void_p()
+        rc = getattr(self.ctx.lib, self._prefix + "create")(self.ctx.h, self.batch, C.byref(cfg), C.byref(h))
+        if rc != 0:
+            raise _lib.B200VOError(f"{self._prefix}create failed ({rc}): {self.ctx.last_error()}")
+        self.h = h
+        if K_rows is not None:
+            self.set_intrinsics(np.arange(self.batch), K_rows)
+        if frame_size is not None:
+            self.set_frame_size(np.arange(self.batch), frame_size)
+        if dist_coeffs is not None:
+            self.set_distortion(np.arange(self.batch), dist_coeffs)
+
+    def close(self):
+        """Destroys the device-side object.  Page-locked arrays handed out by this object (step() results,
+        pinned_empty / pinned_frames) stay valid for as long as they are referenced: each block is owned by its arrays
+        (_PinnedBlock) and released with the last of them."""
+        if getattr(self, "h", None):
+            getattr(self.ctx.lib, self._prefix + "destroy")(self.h)
+            self.h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def _call(self, name, *args):
+        """``<prefix><name>(h, *args)``: a refused argument (-1) raises ValueError, any other failure B200VOError."""
+        what = self._prefix + name
+        rc = getattr(self.ctx.lib, what)(self.h, *args)
+        if rc == -1:
+            raise ValueError(f"{what}: {self.ctx.last_error()}")
+        if rc != 0:
+            raise _lib.B200VOError(f"{what} failed ({rc}): {self.ctx.last_error()}")
+
+    def _seqs(self, seqs) -> np.ndarray:
+        """The sequences of a call as int32 (n,); ValueError unless they are 1 to batch distinct indices in [0, batch)."""
+        a = np.asarray(seqs)
+        if a.ndim != 1 or a.size < 1 or a.size > self.batch or not np.issubdtype(a.dtype, np.integer):
+            raise ValueError(f"seqs must be 1 to batch = {self.batch} integer sequence indices, got {a.dtype} {a.shape}")
+        if ((a < 0) | (a >= self.batch)).any():
+            raise ValueError(f"seqs must lie in [0, batch = {self.batch})")
+        if len(np.unique(a)) != len(a):
+            raise ValueError("seqs must be distinct")
+        return np.ascontiguousarray(a, np.int32)
+
+    def pinned_empty(self, shape, dtype) -> np.ndarray:
+        """numpy array in page-locked host memory (b200vo_host_alloc): DMA'd in place by step()."""
+        dt = np.dtype(dtype)
+        return _PinnedBlock(self.ctx, max(int(np.prod(shape)) * dt.itemsize, 1)).array(shape, dt)
+
+    def pinned_frames(self, n_sets: int = 1) -> np.ndarray:
+        """(n_sets, batch, rows, cols) uint8 array in page-locked memory (b200vo_host_alloc), for submit_frames() and step()."""
+        return self.pinned_empty((n_sets, self.batch, self.rows, self.cols), np.uint8)
+
+    def set_intrinsics(self, seqs, K):
+        """Give the distinct sequences ``seqs`` the camera matrices ``K`` (len(seqs), 3, 3); everything later that poses,
+        triangulates or undistorts those sequences uses their own K.  A K must be a pinhole camera: fx, fy finite and > 0,
+        cx, cy finite, zero skew and other off-diagonal entries, last row (0, 0, 1).  A sequence with distortion keeps its
+        coefficients and gets a new map; its K cannot change while submitted frames wait.  Bad shapes, indices or matrices
+        raise ValueError and change nothing.  Synchronous."""
+        seqs = np.ascontiguousarray(seqs, np.int32).reshape(-1)
+        K = np.ascontiguousarray(K, np.float64)
+        if K.shape != (len(seqs), 3, 3):
+            raise ValueError(f"K must be (len(seqs) = {len(seqs)}, 3, 3), got {K.shape}")
+        self._call("set_intrinsics", len(seqs), _p(seqs, c_i32p), _p(K, c_f64p))
+
+    def set_frame_size(self, seqs, sizes):
+        """Give the distinct sequences ``seqs`` the frame sizes ``sizes`` (len(seqs), 2) int (rows, cols).  ``rows`` x ``cols`` of the
+        constructor is the slot, the largest frame: a sequence's image is the top-left of its slot in every frame array (which
+        may also be a list of per-sequence images), and each sequence runs exactly as in a batch of its own size.  A size must
+        fit the slot and exceed the window.  The listed sequences lose their detection masks and keep their distortion, with
+        new maps.  Bad shapes, indices or sizes, or submitted frames still waiting, raise ValueError and change nothing.
+        Synchronous."""
+        seqs = np.ascontiguousarray(seqs, np.int32).reshape(-1)
+        sizes = np.asarray(sizes)
+        if sizes.shape != (len(seqs), 2) or not np.issubdtype(sizes.dtype, np.integer):
+            raise ValueError(f"sizes must be integer (len(seqs) = {len(seqs)}, 2) (rows, cols), got {sizes.dtype} {sizes.shape}")
+        rows = np.ascontiguousarray(sizes[:, 0], np.int32)
+        cols = np.ascontiguousarray(sizes[:, 1], np.int32)
+        self._call("set_frame_size", len(seqs), _p(seqs, c_i32p), _p(rows, c_i32p), _p(cols, c_i32p))
+        self.frame_size[seqs] = np.stack([rows, cols], 1)
+        self.has_mask[seqs] = False
+
+    def set_detection_mask(self, seqs, masks):
+        """Give the distinct sequences ``seqs`` detection masks (cv2's ``mask=``), e.g. for static regions whose corners move
+        with the camera (a car's hood, the black wedges of an undistorted image, a burned-in timestamp).  ``masks`` is
+        (len(seqs), rows, cols) uint8 in the slot layout (a sequence's mask is the top-left of its row, at its frame size), or a
+        list of per-sequence 2-D uint8 masks at each sequence's frame size; None clears the listed sequences' masks.  A mask
+        gates detection only, as ``cv2_compat.good_features_to_track_masked`` does on the sequence's frame.  Bad shapes, dtypes
+        or indices raise ValueError and change nothing.  Synchronous."""
+        seqs = self._seqs(seqs)
+        if masks is not None:
+            if isinstance(masks, (list, tuple)):
+                masks = _pack_frames(list(masks), self.frame_size[seqs], self.rows, self.cols)
+            masks = np.asarray(masks)
+            if masks.dtype != np.uint8 or masks.shape != (len(seqs), self.rows, self.cols):
+                raise ValueError(f"masks must be ({len(seqs)}, {self.rows}, {self.cols}) uint8 or a list of {len(seqs)} masks, "
+                                 f"got {masks.dtype} {masks.shape}")
+            masks = np.ascontiguousarray(masks)
+        self._call("set_detection_mask", len(seqs), _p(seqs, c_i32p), None if masks is None else _p(masks, c_u8p))
+        self.has_mask[seqs] = masks is not None
+
+    def set_distortion(self, seqs, dist):
+        """Give the distinct sequences ``seqs`` lens distortion: ``dist`` (len(seqs), n) with n = 4, 5 or 8 coefficients in cv2's
+        order (k1, k2, p1, p2[, k3[, k4, k5, k6]]), or None to clear it; an all-zero row clears it too.  Every frame of a
+        sequence with distortion is raw camera output, undistorted on the device as ``cv2.undistort(frame, K, dist)`` does
+        (``cv2_compat.undistort``) before anything reads it: points, poses, states, detected corners and detection masks are in
+        the undistorted image, whose camera is the sequence's K.  ``set_intrinsics`` and ``set_frame_size`` keep the
+        coefficients and rebuild the map.  Bad shapes, non-finite coefficients, bad indices or submitted frames still waiting
+        raise ValueError (the 12- and 14-coefficient models NotImplementedError) and change nothing.  Synchronous."""
+        seqs = self._seqs(seqs)
+        d8 = np.zeros((len(seqs), 8), np.float64)
+        if dist is not None:
+            d = np.asarray(dist)
+            if d.ndim == 2 and d.shape[0] == len(seqs) and d.shape[1] in (12, 14):
+                raise NotImplementedError("the thin-prism (12) and tilted (14) distortion models are not supported")
+            if d.ndim != 2 or d.shape[0] != len(seqs) or d.shape[1] not in (4, 5, 8) or not np.issubdtype(d.dtype, np.number):
+                raise ValueError(f"dist must be (len(seqs) = {len(seqs)}, 4 | 5 | 8) coefficients or None, got {d.dtype} {d.shape}")
+            d8[:, :d.shape[1]] = d
+        self._call("set_distortion", len(seqs), _p(seqs, c_i32p), _p(d8, c_f64p))
+        self.dist_coeffs[seqs] = d8
+
+
+class SequenceBatch(_Batch):
+    """The tracker and pose chain of ``batch`` sequences (``b200vo_batch_*``), host state kept by the caller: ``prime``
+    loads the first frames, every ``step`` tracks the given points into the next frames and poses them.
+
+    ``set_frame_size`` and ``set_distortion`` leave the resident pyramids built from the old sizes or maps: the next step
+    needs ``prime()``.  A detection mask gates ``good_features``."""
+
+    def __init__(self, batch, rows, cols, K, win=(15, 15), max_level=5, criteria=(3, 50, 0.01),
+                 min_eig_thr=1e-4, pnp_iters=500, pnp_reproj_err=8.0, pnp_conf=0.99,
+                 max_landmarks=1024, max_candidates=1024, frame_size=None, dist_coeffs=None, ctx: _lib.Context | None = None):
+        super().__init__("b200vo_batch_", batch, rows, cols, ctx)
+        self.L, self.Cn = int(max_landmarks), int(max_candidates)
         cfg = BatchCfg()
         cfg.rows, cfg.cols = self.rows, self.cols
         cfg.win_w, cfg.win_h, cfg.max_level = int(win[0]), int(win[1]), int(max_level)
@@ -181,18 +250,7 @@ class SequenceBatch:
         for i in range(9):
             cfg.K[i] = float(Kf[i])
         cfg.max_landmarks, cfg.max_candidates = self.L, self.Cn
-        self.cfg = cfg
-        h = C.c_void_p()
-        rc = self.ctx.lib.b200vo_batch_create(self.ctx.h, self.batch, C.byref(cfg), C.byref(h))
-        if rc != 0:
-            raise _lib.B200VOError(f"b200vo_batch_create failed ({rc}): {self.ctx.last_error()}")
-        self.h = h
-        if K_rows is not None:
-            self.set_intrinsics(np.arange(self.batch), K_rows)
-        if frame_size is not None:
-            self.set_frame_size(np.arange(self.batch), frame_size)
-        if dist_coeffs is not None:
-            self.set_distortion(np.arange(self.batch), dist_coeffs)
+        self._create(cfg, K_rows, frame_size, dist_coeffs)
         # host outputs (reused, page-locked so that step() reads them back without a staging copy)
         b, L, Cn = self.batch, self.L, self.Cn
         self.lm_next = self.pinned_empty((b, L, 2), np.float32)
@@ -209,82 +267,18 @@ class SequenceBatch:
         self._out_dict = dict(lm_next=self.lm_next, lm_status=self.lm_status, cand_next=self.cand_next, cand_status=self.cand_status,
                               pose=self.pose, pnp_ok=self.pnp_ok, inlier_mask=self.inlier_mask, n_inliers=self.n_inliers)
 
-    def close(self):
-        """Destroys the device-side batch.  Page-locked arrays handed out by this object (step() results,
-        pinned_empty / pinned_like / pinned_frames) stay valid for as long as they are referenced: each block is
-        owned by its arrays (_PinnedBlock) and released with the last of them."""
-        if getattr(self, "h", None):
-            self.ctx.lib.b200vo_batch_destroy(self.h)
-            self.h = None
-
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:
-            pass
-
     def _chk(self, rc, what):
         if rc != 0:
             raise _lib.B200VOError(f"{what} failed ({rc}): {self.ctx.last_error()}")
-
-    def set_intrinsics(self, seqs, K):
-        """Give the distinct sequences ``seqs`` the camera matrices ``K`` (len(seqs), 3, 3); every later step poses them with
-        their own K.  A K must be a pinhole camera: fx, fy finite and > 0, cx, cy finite, zero skew and other off-diagonal
-        entries, last row (0, 0, 1).  Bad shapes, indices or matrices raise ValueError and change nothing.  Synchronous."""
-        _set_intrinsics(self.ctx, self.ctx.lib.b200vo_batch_set_intrinsics, self.h, self.batch, seqs, K, "b200vo_batch_set_intrinsics")
-
-    def set_frame_size(self, seqs, sizes):
-        """Give the distinct sequences ``seqs`` the frame sizes ``sizes`` (len(seqs), 2) int (rows, cols).  ``rows`` x ``cols`` of the
-        constructor is the slot, the largest frame: a sequence's image is the top-left of its slot in every frame array, and it is
-        tracked and detected exactly as in a batch of its own size.  A size must fit the slot and exceed the window.  Bad shapes,
-        indices or sizes, or submitted frames still waiting, raise ValueError and change nothing.  The next step needs prime().
-        Synchronous."""
-        seqs, sizes = _set_frame_size(self.ctx, self.ctx.lib.b200vo_batch_set_frame_size, self.h, seqs, sizes, "b200vo_batch_set_frame_size")
-        self.frame_size[seqs] = sizes
-        self.has_mask[seqs] = False
-
-    def set_detection_mask(self, seqs, masks):
-        """Give the distinct sequences ``seqs`` detection masks (cv2's ``goodFeaturesToTrack(..., mask=)``): ``masks`` is
-        (len(seqs), rows, cols) uint8 in the slot layout (a sequence's mask is the top-left of its row, at its frame size), or a
-        list of per-sequence 2-D uint8 masks at each sequence's frame size; None clears the listed sequences' masks.
-        ``good_features`` then detects in a masked sequence as ``cv2_compat.good_features_to_track_masked`` does on its frame.
-        ``set_frame_size`` clears the listed sequences' masks.  Bad shapes, dtypes or indices raise ValueError and change
-        nothing.  Synchronous."""
-        seqs = _set_detection_mask(self.ctx, self.ctx.lib.b200vo_batch_set_detection_mask, self.h, self.batch, self.frame_size,
-                                   self.rows, self.cols, seqs, masks, "b200vo_batch_set_detection_mask")
-        self.has_mask[seqs] = masks is not None
-
-    def set_distortion(self, seqs, dist):
-        """Give the distinct sequences ``seqs`` lens distortion: ``dist`` (len(seqs), n) with n = 4, 5 or 8 coefficients in cv2's
-        order (k1, k2, p1, p2[, k3[, k4, k5, k6]]), or None to clear it; an all-zero row clears it too.  Every frame of a
-        sequence with distortion is raw camera output that the batch undistorts on the device as ``cv2.undistort(frame, K,
-        dist)`` does (``cv2_compat.undistort``) before anything reads it: points, poses, ``good_features`` and detection masks
-        are in the undistorted image, whose camera is the sequence's K.  ``set_intrinsics`` and ``set_frame_size`` keep the
-        coefficients and rebuild the map.  Bad shapes, non-finite coefficients, bad indices or submitted frames still waiting
-        raise ValueError (the 12- and 14-coefficient models NotImplementedError) and change nothing.  The next step needs
-        prime().  Synchronous."""
-        seqs, d8 = _set_distortion(self.ctx, self.ctx.lib.b200vo_batch_set_distortion, self.h, self.batch, seqs, dist,
-                                   "b200vo_batch_set_distortion")
-        self.dist_coeffs[seqs] = d8
 
     def _frames(self, frames):
         """frames of a step: the slot-layout array, or a list of per-sequence 2-D images packed into it"""
         return _pack_frames(frames, self.frame_size, self.rows, self.cols)
 
-    def pinned_empty(self, shape, dtype) -> np.ndarray:
-        """numpy array in page-locked host memory (b200vo_host_alloc): DMA'd in place by step()."""
-        dt = np.dtype(dtype)
-        nbytes = max(int(np.prod(shape)) * dt.itemsize, 1)
-        return _PinnedBlock(self.ctx, nbytes).array(shape, dt)
-
     def pinned_like(self, arr: np.ndarray) -> np.ndarray:
         out = self.pinned_empty(arr.shape, arr.dtype)
         out[...] = arr
         return out
-
-    def pinned_frames(self, n_sets: int = 1) -> np.ndarray:
-        """(n_sets, batch, rows, cols) uint8 array in page-locked memory (b200vo_host_alloc)."""
-        return self.pinned_empty((n_sets, self.batch, self.rows, self.cols), np.uint8)
 
     def prime(self, frames):
         frames = np.ascontiguousarray(self._frames(frames), np.uint8).reshape(self.batch, self.rows, self.cols)
@@ -374,7 +368,7 @@ def _loop_cfg(rows, cols, K, options, max_landmarks, max_candidates, max_frames)
     return cfg
 
 
-class VOBatch:
+class VOBatch(_Batch):
     """The whole per-frame loop of the reference (``continuous_operation``, ``VisualOdometryPipeLine.py:326-373``) for
     ``batch`` independent sequences, with the VO state of every sequence resident on the device (``b200vo_loop_*``).
 
@@ -387,33 +381,23 @@ class VOBatch:
     device instead of ``load``; a sequence whose bootstrap finds no essential matrix gets ``NO_BOOTSTRAP``.
 
     ``K`` is the camera matrix of every sequence, (3, 3), or one per sequence, (batch, 3, 3).  ``set_intrinsics`` (or the
-    ``K`` argument of ``load`` / ``bootstrap``) gives a slot another camera, e.g. when it is handed to a new sequence."""
+    ``K`` argument of ``load`` / ``bootstrap``) gives a slot another camera, e.g. when it is handed to a new sequence: it
+    does not touch the sequences' states, status and frames, so set a K just before ``load`` or ``bootstrap``.
+    ``set_frame_size`` and ``set_distortion`` make the listed sequences IDLE (state kept, skipped by ``step``) until
+    ``load`` or ``bootstrap``.  The frames of ``step``, ``submit_frames``, ``load`` and ``bootstrap`` follow each
+    sequence's frame size and distortion.  A detection mask gates the corners a step adds (as
+    ``cv2_compat.good_features_to_track_masked``) and both SIFT frames of ``bootstrap`` (as ``match_bootstrap_frames(...,
+    mask=)``); tracking, pose and triangulation do not read it."""
 
     OK, IDLE, FEW_POINTS, PNP_FAILED, OVERFLOW, DETECT_LIMIT, NO_BOOTSTRAP = range(7)
 
     def __init__(self, batch, rows, cols, K, options, max_landmarks=4096, max_candidates=8192, max_frames=1024,
                  frame_size=None, dist_coeffs=None, ctx: _lib.Context | None = None):
-        self.ctx = ctx or _lib.default_context(0)
-        self.batch, self.rows, self.cols = int(batch), int(rows), int(cols)
-        self.frame_size = np.tile(np.int32([self.rows, self.cols]), (self.batch, 1))   # (batch, 2) rows, cols of every sequence
-        self.has_mask = np.zeros(self.batch, bool)   # the sequences with a detection mask (set_detection_mask)
-        self.dist_coeffs = np.zeros((self.batch, 8))   # k1, k2, p1, p2, k3, k4, k5, k6 of every sequence (set_distortion)
-        self._submitted = []
+        super().__init__("b200vo_loop_", batch, rows, cols, ctx)
         self.L, self.Cn, self.P = int(max_landmarks), int(max_candidates), int(max_frames)
         self.options = options
         K, K_rows = _batch_K(K, self.batch)
-        self.cfg = _loop_cfg(rows, cols, K, options, max_landmarks, max_candidates, max_frames)
-        h = C.c_void_p()
-        rc = self.ctx.lib.b200vo_loop_create(self.ctx.h, self.batch, C.byref(self.cfg), C.byref(h))
-        if rc != 0:
-            raise _lib.B200VOError(f"b200vo_loop_create failed ({rc}): {self.ctx.last_error()}")
-        self.h = h
-        if K_rows is not None:
-            self.set_intrinsics(np.arange(self.batch), K_rows)
-        if frame_size is not None:
-            self.set_frame_size(np.arange(self.batch), frame_size)
-        if dist_coeffs is not None:
-            self.set_distortion(np.arange(self.batch), dist_coeffs)
+        self._create(_loop_cfg(rows, cols, K, options, max_landmarks, max_candidates, max_frames), K_rows, frame_size, dist_coeffs)
         b = self.batch
         self._res = dict(status=self.pinned_empty((b,), np.int32), n_inliers=self.pinned_empty((b,), np.int32),
                          n_lm=self.pinned_empty((b,), np.int32), n_cand=self.pinned_empty((b,), np.int32),
@@ -421,76 +405,6 @@ class VOBatch:
         r = self._res
         self._res_ptrs = (_p(r['status'], c_i32p), _p(r['n_inliers'], c_i32p), _p(r['n_lm'], c_i32p), _p(r['n_cand'], c_i32p),
                           _p(r['pose_cw'], c_f64p))
-
-    def close(self):
-        if getattr(self, "h", None):
-            self.ctx.lib.b200vo_loop_destroy(self.h)
-            self.h = None
-
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:
-            pass
-
-    def _chk(self, rc, what):
-        if rc == -1:
-            raise ValueError(f"{what}: {self.ctx.last_error()}")
-        if rc != 0:
-            raise _lib.B200VOError(f"{what} failed ({rc}): {self.ctx.last_error()}")
-
-    def pinned_empty(self, shape, dtype) -> np.ndarray:
-        """numpy array in page-locked host memory (b200vo_host_alloc)."""
-        dt = np.dtype(dtype)
-        return _PinnedBlock(self.ctx, max(int(np.prod(shape)) * dt.itemsize, 1)).array(shape, dt)
-
-    def pinned_frames(self, n_sets: int = 1) -> np.ndarray:
-        """(n_sets, batch, rows, cols) uint8 array in page-locked memory, for submit_frames() and step()."""
-        return self.pinned_empty((n_sets, self.batch, self.rows, self.cols), np.uint8)
-
-    def set_intrinsics(self, seqs, K):
-        """Give the distinct sequences ``seqs`` the camera matrices ``K`` (len(seqs), 3, 3): every later step and bootstrap of
-        those sequences tracks, poses and triangulates with their own K.  A K must be a pinhole camera: fx, fy finite and > 0,
-        cx, cy finite, zero skew and other off-diagonal entries, last row (0, 0, 1).  The sequences' states, status and frames
-        are not touched: to hand a slot to a sequence of another camera, set its K just before ``load`` or ``bootstrap`` (or
-        pass ``K`` to them).  Bad shapes, indices or matrices raise ValueError and change nothing.  Synchronous."""
-        _set_intrinsics(self.ctx, self.ctx.lib.b200vo_loop_set_intrinsics, self.h, self.batch, seqs, K, "b200vo_loop_set_intrinsics")
-
-    def set_frame_size(self, seqs, sizes):
-        """Give the distinct sequences ``seqs`` the frame sizes ``sizes`` (len(seqs), 2) int (rows, cols).  ``rows`` x ``cols`` of the
-        constructor is the slot, the largest frame: a sequence's image is the top-left of its slot in the frames of ``step``,
-        ``submit_frames`` and ``bootstrap`` (which also take a list of per-sequence images), and each sequence runs exactly as in
-        a batch of its own size.  The listed sequences become IDLE (state kept, skipped by ``step``) until ``load`` or
-        ``bootstrap``.  A size must fit the slot and exceed the window.  Bad shapes, indices or sizes, or submitted frames
-        still waiting, raise ValueError and change nothing.  Synchronous."""
-        seqs, sizes = _set_frame_size(self.ctx, self.ctx.lib.b200vo_loop_set_frame_size, self.h, seqs, sizes, "b200vo_loop_set_frame_size")
-        self.frame_size[seqs] = sizes
-        self.has_mask[seqs] = False
-
-    def set_detection_mask(self, seqs, masks):
-        """Give the distinct sequences ``seqs`` detection masks, for static regions whose corners move with the camera (a car's
-        hood, the black wedges of an undistorted image, a burned-in timestamp).  ``masks``: (len(seqs), rows, cols) uint8 in the
-        slot layout, or a list of per-sequence 2-D uint8 masks at each sequence's frame size; None clears the listed sequences'
-        masks.  A mask gates detection only: the corners a step adds (as ``cv2_compat.good_features_to_track_masked``) and
-        both SIFT frames of ``bootstrap`` (as ``match_bootstrap_frames(..., mask=)``); tracking, pose and triangulation do not
-        read it.  The sequences' states, status and frames are not touched; ``set_frame_size`` clears the listed sequences'
-        masks.  Bad shapes, dtypes or indices raise ValueError and change nothing.  Synchronous."""
-        seqs = _set_detection_mask(self.ctx, self.ctx.lib.b200vo_loop_set_detection_mask, self.h, self.batch, self.frame_size,
-                                   self.rows, self.cols, seqs, masks, "b200vo_loop_set_detection_mask")
-        self.has_mask[seqs] = masks is not None
-
-    def set_distortion(self, seqs, dist):
-        """Give the distinct sequences ``seqs`` lens distortion: ``dist`` (len(seqs), n) with n = 4, 5 or 8 coefficients in cv2's
-        order (k1, k2, p1, p2[, k3[, k4, k5, k6]]), or None to clear it; an all-zero row clears it too.  Every frame the loop
-        takes for such a sequence (``step``, ``submit_frames``, ``load``, both frames of ``bootstrap``) is raw camera output,
-        undistorted on the device as ``cv2.undistort(frame, K, dist)`` does before anything reads it; states, ``read_state``,
-        poses and detection masks are in the undistorted image, whose camera is the sequence's K.  ``set_intrinsics`` and
-        ``set_frame_size`` keep the coefficients and rebuild the map.  The listed sequences become IDLE until ``load`` or
-        ``bootstrap``.  Bad shapes, non-finite coefficients, bad indices or submitted frames still waiting raise ValueError
-        (the 12- and 14-coefficient models NotImplementedError) and change nothing.  Synchronous."""
-        seqs, d8 = _set_distortion(self.ctx, self.ctx.lib.b200vo_loop_set_distortion, self.h, self.batch, seqs, dist,
-                                   "b200vo_loop_set_distortion")
-        self.dist_coeffs[seqs] = d8
 
     def load(self, seq: int, frame: np.ndarray, state: dict, K=None):
         """Set sequence ``seq`` to ``state`` (see the class docstring) with ``frame`` as its current frame; its status
@@ -521,9 +435,8 @@ class VOBatch:
             if not (len(lm) <= self.L and len(keys) <= self.Cn and 1 <= len(poses) <= self.P) or (fp < 0).any() or (fp >= len(poses)).any():
                 raise ValueError("b200vo_loop_load: a count is out of range or a first_pose value outside [0, n_poses)")
             self.set_intrinsics([seq], K[None])
-        self._chk(self.ctx.lib.b200vo_loop_load(self.h, int(seq), _p(f, c_u8p), _p(lm, c_f32p), _p(kp, c_f32p), len(lm),
-                                                _p(keys, c_f32p), _p(fk, c_f32p), _p(fp, c_i32p), len(keys), _p(poses, c_f64p),
-                                                len(poses)), "b200vo_loop_load")
+        self._call("load", int(seq), _p(f, c_u8p), _p(lm, c_f32p), _p(kp, c_f32p), len(lm), _p(keys, c_f32p), _p(fk, c_f32p),
+                   _p(fp, c_i32p), len(keys), _p(poses, c_f64p), len(poses))
         if K is not None and not K_first:   # after the load, which is the call that can still refuse
             self.set_intrinsics([seq], K[None])
 
@@ -553,9 +466,8 @@ class VOBatch:
             self.set_intrinsics(seqs, K)
         n = len(seqs)
         out = {k: np.zeros(max(n, 1), np.int32) for k in ('status', 'num_pts', 'n_lm', 'n_cand')}
-        self._chk(self.ctx.lib.b200vo_loop_bootstrap(self.h, n, _p(seqs, c_i32p), _p(f0, c_u8p), _p(f1, c_u8p),
-                                                     float(self.options['feature_ratio']), *(_p(out[k], c_i32p) for k in out)),
-                  "b200vo_loop_bootstrap")
+        self._call("bootstrap", n, _p(seqs, c_i32p), _p(f0, c_u8p), _p(f1, c_u8p), float(self.options['feature_ratio']),
+                   *(_p(out[k], c_i32p) for k in out))
         return {k: v[:n] for k, v in out.items()}
 
     def read_state(self, seq: int) -> dict:
@@ -567,23 +479,11 @@ class VOBatch:
         fp = np.zeros(self.Cn, np.int32)
         poses = np.zeros((self.P, 12), np.float64)
         n_lm, n_cand, n_poses, status = (C.c_int32(0) for _ in range(4))
-        self._chk(self.ctx.lib.b200vo_loop_read_state(self.h, int(seq), _p(lm, c_f32p), _p(kp, c_f32p), C.byref(n_lm), _p(keys, c_f32p),
-                                                      _p(fk, c_f32p), _p(fp, c_i32p), C.byref(n_cand), _p(poses, c_f64p),
-                                                      C.byref(n_poses), C.byref(status)), "b200vo_loop_read_state")
+        self._call("read_state", int(seq), _p(lm, c_f32p), _p(kp, c_f32p), C.byref(n_lm), _p(keys, c_f32p), _p(fk, c_f32p),
+                   _p(fp, c_i32p), C.byref(n_cand), _p(poses, c_f64p), C.byref(n_poses), C.byref(status))
         nl, nc, npo = n_lm.value, n_cand.value, n_poses.value
         return dict(lm=lm[:nl], lm_kp=kp[:nl], keys=keys[:nc], first_keys=fk[:nc], first_pose=fp[:nc], poses=poses[:npo],
                     status=status.value)
-
-    def _list(self, seqs) -> np.ndarray:
-        """The sequences of a listed step as int32 (n,); ValueError unless they are 1 to batch distinct indices in [0, batch)."""
-        a = np.asarray(seqs)
-        if a.ndim != 1 or a.size < 1 or a.size > self.batch or not np.issubdtype(a.dtype, np.integer):
-            raise ValueError(f"seqs must be 1 to batch = {self.batch} integer sequence indices, got {a.dtype} {a.shape}")
-        if ((a < 0) | (a >= self.batch)).any():
-            raise ValueError(f"seqs must lie in [0, batch = {self.batch})")
-        if len(np.unique(a)) != len(a):
-            raise ValueError("seqs must be distinct")
-        return np.ascontiguousarray(a, np.int32)
 
     def _listed_frames(self, frames, seqs, out=None) -> np.ndarray:
         """frames of a listed step: (len(seqs), rows, cols) uint8 in the slot layout, or a list of the listed sequences' images"""
@@ -597,30 +497,28 @@ class VOBatch:
         copy); step(None) consumes them, oldest first.  ``seqs``: the frames of a listed step (see ``step``), consumed by
         ``step(None, seqs)`` with the same list."""
         if seqs is not None:
-            seqs = self._list(seqs)
+            seqs = self._seqs(seqs)
             if isinstance(frames, (list, tuple)):
                 frames = self._listed_frames(frames, seqs, self.pinned_empty((len(seqs), self.rows, self.cols), np.uint8))
                 self._submitted = (self._submitted + [frames])[-3:]
             else:
                 frames = self._listed_frames(frames, seqs)
-            self._chk(self.ctx.lib.b200vo_loop_submit_frames_seqs(self.h, len(seqs), _p(seqs, c_i32p), _p(frames, c_u8p)),
-                      "b200vo_loop_submit_frames_seqs")
+            self._call("submit_frames_seqs", len(seqs), _p(seqs, c_i32p), _p(frames, c_u8p))
             return
         if isinstance(frames, (list, tuple)):
             frames = _pack_frames(frames, self.frame_size, self.rows, self.cols, self.pinned_frames()[0])
             self._submitted = (self._submitted + [frames])[-3:]
         assert frames.dtype == np.uint8 and frames.flags.c_contiguous and frames.size == self.batch * self.rows * self.cols
-        self._chk(self.ctx.lib.b200vo_loop_submit_frames(self.h, _p(frames, c_u8p)), "b200vo_loop_submit_frames")
+        self._call("submit_frames", _p(frames, c_u8p))
 
     def submit_frames_dev(self, frames_dev: int, seqs=None):
         """The same for frames resident in device memory (int from tensor.data_ptr()); step_dev(None, ...) consumes them.
         ``seqs``: (len(seqs), rows, cols) frames of a listed step, consumed by ``step_dev(None, out_dev, seqs)``."""
         if seqs is not None:
-            seqs = self._list(seqs)
-            self._chk(self.ctx.lib.b200vo_loop_submit_frames_seqs_dev(self.h, len(seqs), _p(seqs, c_i32p), frames_dev),
-                      "b200vo_loop_submit_frames_seqs_dev")
+            seqs = self._seqs(seqs)
+            self._call("submit_frames_seqs_dev", len(seqs), _p(seqs, c_i32p), frames_dev)
             return
-        self._chk(self.ctx.lib.b200vo_loop_submit_frames_dev(self.h, frames_dev), "b200vo_loop_submit_frames_dev")
+        self._call("submit_frames_dev", frames_dev)
 
     def step(self, frames=None, seqs=None) -> dict:
         """One frame for every sequence (frames (batch, rows, cols) uint8 in the slot layout, or a list of per-sequence images;
@@ -634,18 +532,16 @@ class VOBatch:
         batch of its own; the others are not touched and resume from their current frame when they are listed again.  The
         results are the first len(seqs) rows of the same arrays, in list order.  Bad shapes or indices raise ValueError."""
         if seqs is not None:
-            seqs = self._list(seqs)
+            seqs = self._seqs(seqs)
             n = len(seqs)
             if frames is not None:
                 frames = self._listed_frames(frames, seqs)
-            self._chk(self.ctx.lib.b200vo_loop_step_seqs(self.h, n, _p(seqs, c_i32p), _p(frames, c_u8p) if frames is not None else None,
-                                                         *self._res_ptrs), "b200vo_loop_step_seqs")
+            self._call("step_seqs", n, _p(seqs, c_i32p), _p(frames, c_u8p) if frames is not None else None, *self._res_ptrs)
             return {k: v[:n] for k, v in self._res.items()}
         if frames is not None:
             frames = np.ascontiguousarray(_pack_frames(frames, self.frame_size, self.rows, self.cols), np.uint8)
             assert frames.size == self.batch * self.rows * self.cols
-        self._chk(self.ctx.lib.b200vo_loop_step(self.h, _p(frames, c_u8p) if frames is not None else None, *self._res_ptrs),
-                  "b200vo_loop_step")
+        self._call("step", _p(frames, c_u8p) if frames is not None else None, *self._res_ptrs)
         return self._res
 
     def step_dev(self, frames_dev, out_dev: dict, seqs=None):
@@ -655,13 +551,11 @@ class VOBatch:
         and the results fill the first len(seqs) rows in list order."""
         o = out_dev
         if seqs is not None:
-            seqs = self._list(seqs)
-            self._chk(self.ctx.lib.b200vo_loop_step_seqs_dev(self.h, len(seqs), _p(seqs, c_i32p), frames_dev or None, o['status'],
-                                                             o['n_inliers'], o['n_lm'], o['n_cand'], o['pose_cw']),
-                      "b200vo_loop_step_seqs_dev")
+            seqs = self._seqs(seqs)
+            self._call("step_seqs_dev", len(seqs), _p(seqs, c_i32p), frames_dev or None, o['status'], o['n_inliers'], o['n_lm'],
+                       o['n_cand'], o['pose_cw'])
             return
-        self._chk(self.ctx.lib.b200vo_loop_step_dev(self.h, frames_dev or None, o['status'], o['n_inliers'], o['n_lm'], o['n_cand'],
-                                                    o['pose_cw']), "b200vo_loop_step_dev")
+        self._call("step_dev", frames_dev or None, o['status'], o['n_inliers'], o['n_lm'], o['n_cand'], o['pose_cw'])
 
 
 def match_bootstrap_frames(frame0, frame1, ratio=0.8, mask=None):

@@ -50,6 +50,109 @@ scatter_mask_kernel(int cap, const uint8_t* __restrict__ ok, const int* __restri
     if (threadIdx.x == 0) { n_inl_out[b] = m; ok_out[b] = ok[b]; }
 }
 
+enum VoSetting { VO_SET_INTRINSICS, VO_SET_FRAME_SIZE, VO_SET_DISTORTION, VO_SET_MASK };
+
+// What a new setting of the listed sequences does besides writing their rows.  A submitted frame set's pyramids were built
+// (and undistorted) with the settings of its submission: `waiting` is the refusal while one waits (nullptr: never refused;
+// only_distorted: only when a listed sequence has distortion, the one use of K in a pyramid).  stale: the listed sequences'
+// resident pyramids no longer match their frames.  unmask: a mask has its sequence's frame size, so the listed sequences
+// lose theirs.  remap: a map depends on K, the coefficients and the frame size, so the listed sequences with distortion
+// get new maps (their coefficients kept).
+static const struct { const char* waiting; bool only_distorted, stale, unmask, remap; } k_setting[] = {
+    /* intrinsics */     {"submitted frame sets are waiting: their pyramids were undistorted with the old K", true, false, false, true},
+    /* frame size */     {"submitted frame sets are waiting: their pyramids were built at the old sizes", false, true, true, true},
+    /* distortion */     {"submitted frame sets are waiting: their pyramids were built with the old maps", false, true, false, true},
+    /* detection mask */ {nullptr, false, false, false, false},
+};
+
+// the map of every listed sequence with distortion, from its K, coefficients and frame size (the work in flight has ended)
+static int batch_build_maps(b200vo_batch* B, int n_seq, const int32_t* seqs)
+{
+    b200vo_ctx* ctx = B->ctx;
+    const b200vo_batch_cfg& c = B->cfg;
+    std::vector<double> par;
+    std::vector<int32_t> im;
+    for (int k = 0; k < n_seq; ++k) {
+        const int s = seqs[k];
+        const VoSeqSettings& q = B->seq[s];
+        if (!q.distorted()) continue;
+        const VoIntrinsics& r = q.intr;
+        const double* d = q.dist;
+        const double row[14] = {r.fx, r.fy, r.cx, r.cy, d[0], d[1], d[2], d[3], d[4], d[5], d[6], d[7],
+                                (double)q.ext.w[0], (double)q.ext.h[0]};
+        par.insert(par.end(), row, row + 14);
+        im.push_back(s);
+    }
+    if (im.empty()) return 0;
+    const size_t n = im.size(), b_par = vo_align(n * 14 * sizeof(double), 256), fb = (size_t)c.rows * c.cols;
+    VO_TRY(vo_reserve(ctx, B->dist_par, b_par + n * 4));
+    uint8_t* p = (uint8_t*)B->dist_par.p;
+    VO_CUDA(ctx, cudaMemcpyAsync(p, par.data(), par.size() * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+    VO_CUDA(ctx, cudaMemcpyAsync(p + b_par, im.data(), n * 4, cudaMemcpyHostToDevice, ctx->stream));
+    uint8_t* m = (uint8_t*)B->dist_buf.p + vo_align((size_t)B->batch, 256);
+    VO_TRY(vo_undistort_maps(ctx, (const double*)p, (const int*)(p + b_par), (int)n, c.rows, c.cols, (short2*)m,
+                             (uint16_t*)(m + (size_t)B->batch * fb * 4), fb, c.cols, ctx->stream));
+    VO_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    return 0;
+}
+
+// The one update path of the settings: `next` is the table with the listed sequences' new rows (their inputs checked).
+// Refuses as k_setting says, waits for the work in flight, uploads the rows and flags (and the listed sequences' masks
+// from `masks`), then takes `next` as the table and rebuilds maps.  Nothing changes on a refusal.  Synchronous.
+static int batch_apply(b200vo_batch* B, VoSetting kind, std::vector<VoSeqSettings>& next, int n_seq, const int32_t* seqs,
+                       const uint8_t* masks, bool* stale)
+{
+    b200vo_ctx* ctx = B->ctx;
+    const b200vo_batch_cfg& c = B->cfg;
+    const int nb = B->batch;
+    const auto& rule = k_setting[kind];
+    bool listed_dist = false;
+    for (int k = 0; k < n_seq; ++k) listed_dist = listed_dist || next[seqs[k]].distorted();
+    if (rule.waiting && B->q_count > 0 && (!rule.only_distorted || listed_dist)) return vo_set_err(ctx, B200VO_E_BADARG, "%s", rule.waiting);
+    if (rule.unmask)
+        for (int k = 0; k < n_seq; ++k) next[seqs[k]].mask = false;
+    std::vector<VoIntrinsics> intr(nb);
+    std::vector<VoSeqExt> ext(nb);
+    std::vector<uint8_t> mask_flag(nb), dist_flag(nb);
+    int n_mask = 0, n_dist = 0;
+    bool uniform = true;
+    for (int s = 0; s < nb; ++s) {
+        intr[s] = next[s].intr;
+        ext[s] = next[s].ext;
+        mask_flag[s] = next[s].mask;
+        dist_flag[s] = next[s].distorted();
+        n_mask += mask_flag[s];
+        n_dist += dist_flag[s];
+        uniform = uniform && ext[s].w[0] == c.cols && ext[s].h[0] == c.rows;
+    }
+    const size_t fb = (size_t)c.rows * c.cols, b_on = vo_align((size_t)nb, 256);
+    VO_CUDA(ctx, cudaSetDevice(ctx->device));
+    VO_CUDA(ctx, cudaStreamSynchronize(ctx->stream));   // no step in flight reads the settings (every stream of a step joins the ctx stream)
+    VO_CUDA(ctx, cudaStreamSynchronize(B->pre_stream)); // nor the pyramid build of a submitted set
+    VO_TRY(vo_reserve(ctx, B->intr_buf, (size_t)nb * sizeof(VoIntrinsics)));
+    VO_TRY(vo_reserve(ctx, B->ext_buf, (size_t)nb * sizeof(VoSeqExt)));
+    if (n_mask) VO_TRY(vo_reserve(ctx, B->mask_buf, b_on + nb * fb));
+    if (n_dist) VO_TRY(vo_reserve(ctx, B->dist_buf, b_on + nb * fb * 6));
+    VO_CUDA(ctx, cudaMemcpyAsync(B->intr_buf.p, intr.data(), intr.size() * sizeof(VoIntrinsics), cudaMemcpyHostToDevice, ctx->stream));
+    VO_CUDA(ctx, cudaMemcpyAsync(B->ext_buf.p, ext.data(), ext.size() * sizeof(VoSeqExt), cudaMemcpyHostToDevice, ctx->stream));
+    if (B->mask_buf.p) {
+        uint8_t* d = (uint8_t*)B->mask_buf.p;
+        for (int k = 0; masks && k < n_seq; ++k)
+            VO_CUDA(ctx, cudaMemcpyAsync(d + b_on + seqs[k] * fb, masks + k * fb, fb, cudaMemcpyHostToDevice, ctx->stream));
+        VO_CUDA(ctx, cudaMemcpyAsync(d, mask_flag.data(), nb, cudaMemcpyHostToDevice, ctx->stream));
+    }
+    if (B->dist_buf.p) VO_CUDA(ctx, cudaMemcpyAsync(B->dist_buf.p, dist_flag.data(), nb, cudaMemcpyHostToDevice, ctx->stream));
+    VO_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    B->seq.swap(next);
+    B->n_mask = n_mask;
+    B->n_dist = n_dist;
+    B->intr = (const VoIntrinsics*)B->intr_buf.p;
+    B->ext = uniform ? nullptr : (const VoSeqExt*)B->ext_buf.p;
+    if (rule.remap) VO_TRY(batch_build_maps(B, n_seq, seqs));
+    *stale = rule.stale;
+    return 0;
+}
+
 extern "C" int b200vo_batch_create(b200vo_ctx* ctx, int batch, const b200vo_batch_cfg* cfg, b200vo_batch** out)
 {
     if (!ctx || !cfg || !out || batch <= 0) return B200VO_E_BADARG;
@@ -111,103 +214,40 @@ extern "C" int b200vo_batch_create(b200vo_ctx* ctx, int batch, const b200vo_batc
     B->inliers = (int*)p; p += b_i;
     B->c_mask = p; p += b_m;
     B->pnp_ws = p;
-    // every sequence starts with cfg->K
-    B->intr_host.resize(batch);
-    vo_intrinsics_row(B->intr_host[0], cfg->K, VO_BOOT_EMAT_THR);
-    for (int k = 1; k < batch; ++k) B->intr_host[k] = B->intr_host[0];
-    rc = vo_reserve(ctx, B->intr_buf, (size_t)batch * sizeof(VoIntrinsics));
-    if (!rc) {
-        cudaError_t e = cudaMemcpyAsync(B->intr_buf.p, B->intr_host.data(), (size_t)batch * sizeof(VoIntrinsics), cudaMemcpyHostToDevice, ctx->stream);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-        if (e != cudaSuccess) rc = vo_cuda_fail(ctx, e, "b200vo_batch_create: intrinsics upload");
-    }
+    // every sequence starts with cfg->K, the slot size, no mask and no distortion (no mask or map buffer until the first one)
+    std::vector<VoSeqSettings> table(batch, VoSeqSettings{});
+    vo_intrinsics_row(table[0].intr, cfg->K, VO_BOOT_EMAT_THR);
+    vo_seq_ext(cfg->rows, cfg->cols, cfg->win_w, cfg->win_h, cfg->max_level, &table[0].ext);
+    std::vector<int32_t> all(batch, 0);
+    for (int s = 1; s < batch; ++s) { table[s] = table[0]; all[s] = s; }
+    bool stale = false;
+    rc = batch_apply(B, VO_SET_INTRINSICS, table, batch, all.data(), nullptr, &stale);
     if (rc) { b200vo_batch_destroy(B); return rc; }
-    B->intr = (const VoIntrinsics*)B->intr_buf.p;
-    // every sequence starts with the slot size (no table on the device until a sequence is given another)
-    B->ext_host.resize(batch);
-    vo_seq_ext(cfg->rows, cfg->cols, cfg->win_w, cfg->win_h, cfg->max_level, &B->ext_host[0]);
-    for (int k = 1; k < batch; ++k) B->ext_host[k] = B->ext_host[0];
-    rc = vo_reserve(ctx, B->ext_buf, (size_t)batch * sizeof(VoSeqExt));
-    if (rc) { b200vo_batch_destroy(B); return rc; }
-    B->mask_host.assign(batch, 0);   // no masks (and no mask buffer until the first one)
-    B->dist_host.assign((size_t)batch * 8, 0.0);   // no distortion (and no maps until the first one)
-    B->dist_on.assign(batch, 0);
     *out = B;
     return 0;
 }
 
-// the map of every listed sequence with distortion, from its K, coefficients and frame size (the work in flight has ended)
-static int batch_build_maps(b200vo_batch* B, int n_seq, const int32_t* seqs)
+int batch_set_intrinsics(b200vo_batch* B, int n_seq, const int32_t* seqs, const double* K, bool* stale)
+{
+    b200vo_ctx* ctx = B->ctx;
+    VO_TRY(vo_check_seqs(ctx, B->batch, n_seq, seqs));
+    if (!K) return vo_set_err(ctx, B200VO_E_BADARG, "null array");
+    for (int k = 0; k < n_seq; ++k)
+        if (!vo_intrinsics_valid(K + 9 * k))
+            return vo_set_err(ctx, B200VO_E_BADARG, "K[%d] is not a camera matrix: fx, fy finite and > 0, cx, cy finite, "
+                                                    "skew 0, last row (0, 0, 1)", k);
+    std::vector<VoSeqSettings> next = B->seq;
+    for (int k = 0; k < n_seq; ++k) vo_intrinsics_row(next[seqs[k]].intr, K + 9 * k, VO_BOOT_EMAT_THR);
+    return batch_apply(B, VO_SET_INTRINSICS, next, n_seq, seqs, nullptr, stale);
+}
+
+int batch_set_frame_size(b200vo_batch* B, int n_seq, const int32_t* seqs, const int32_t* rows, const int32_t* cols, bool* stale)
 {
     b200vo_ctx* ctx = B->ctx;
     const b200vo_batch_cfg& c = B->cfg;
-    std::vector<double> par;
-    std::vector<int32_t> im;
+    VO_TRY(vo_check_seqs(ctx, B->batch, n_seq, seqs));
+    if (!rows || !cols) return vo_set_err(ctx, B200VO_E_BADARG, "null array");
     for (int k = 0; k < n_seq; ++k) {
-        const int s = seqs[k];
-        if (!B->dist_on[s]) continue;
-        const VoIntrinsics& r = B->intr_host[s];
-        const double* d = B->dist_host.data() + 8 * (size_t)s;
-        const double row[14] = {r.fx, r.fy, r.cx, r.cy, d[0], d[1], d[2], d[3], d[4], d[5], d[6], d[7],
-                                (double)B->ext_host[s].w[0], (double)B->ext_host[s].h[0]};
-        par.insert(par.end(), row, row + 14);
-        im.push_back(s);
-    }
-    if (im.empty()) return 0;
-    const size_t n = im.size(), b_par = vo_align(n * 14 * sizeof(double), 256), fb = (size_t)c.rows * c.cols;
-    VO_TRY(vo_reserve(ctx, B->dist_par, b_par + n * 4));
-    uint8_t* p = (uint8_t*)B->dist_par.p;
-    VO_CUDA(ctx, cudaMemcpyAsync(p, par.data(), par.size() * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
-    VO_CUDA(ctx, cudaMemcpyAsync(p + b_par, im.data(), n * 4, cudaMemcpyHostToDevice, ctx->stream));
-    uint8_t* m = (uint8_t*)B->dist_buf.p + vo_align((size_t)B->batch, 256);
-    VO_TRY(vo_undistort_maps(ctx, (const double*)p, (const int*)(p + b_par), (int)n, c.rows, c.cols, (short2*)m,
-                             (uint16_t*)(m + (size_t)B->batch * fb * 4), fb, c.cols, ctx->stream));
-    VO_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    return 0;
-}
-
-static bool batch_any_dist(const b200vo_batch* B, int n_seq, const int32_t* seqs)
-{
-    bool any = false;
-    for (int k = 0; k < n_seq; ++k) any = any || (seqs[k] >= 0 && seqs[k] < B->batch && B->dist_on[seqs[k]]);
-    return any;
-}
-
-int batch_set_intrinsics(b200vo_batch* B, int n_seq, const int32_t* seqs, const double* K)
-{
-    b200vo_ctx* ctx = B->ctx;
-    std::vector<VoIntrinsics> rows = B->intr_host;
-    VO_TRY(vo_intrinsics_set(ctx, B->batch, n_seq, seqs, K, VO_BOOT_EMAT_THR, rows.data()));
-    // a sequence with distortion undistorts its frames with K: the submitted sets were built with the old one
-    const bool remap = batch_any_dist(B, n_seq, seqs);
-    if (remap && B->q_count > 0)
-        return vo_set_err(ctx, B200VO_E_BADARG, "submitted frame sets are waiting: their pyramids were undistorted with the old K");
-    VO_CUDA(ctx, cudaSetDevice(ctx->device));
-    VO_CUDA(ctx, cudaStreamSynchronize(ctx->stream));   // no step in flight reads the rows (every stream of a step joins the ctx stream)
-    if (remap) VO_CUDA(ctx, cudaStreamSynchronize(B->pre_stream));
-    VO_CUDA(ctx, cudaMemcpyAsync(B->intr_buf.p, rows.data(), rows.size() * sizeof(VoIntrinsics), cudaMemcpyHostToDevice, ctx->stream));
-    VO_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    B->intr_host.swap(rows);
-    if (remap) VO_TRY(batch_build_maps(B, n_seq, seqs));
-    return 0;
-}
-
-extern "C" int b200vo_batch_set_intrinsics(b200vo_batch* B, int n_seq, const int32_t* seqs, const double* K)
-{
-    return B ? batch_set_intrinsics(B, n_seq, seqs, K) : B200VO_E_BADARG;
-}
-
-int batch_set_frame_size(b200vo_batch* B, int n_seq, const int32_t* seqs, const int32_t* rows, const int32_t* cols)
-{
-    b200vo_ctx* ctx = B->ctx;
-    const b200vo_batch_cfg& c = B->cfg;
-    if (n_seq < 1 || n_seq > B->batch) return vo_set_err(ctx, B200VO_E_BADARG, "n_seq = %d is outside [1, batch = %d]", n_seq, B->batch);
-    if (!seqs || !rows || !cols) return vo_set_err(ctx, B200VO_E_BADARG, "null array");
-    std::vector<char> seen(B->batch, 0);
-    for (int k = 0; k < n_seq; ++k) {
-        if (seqs[k] < 0 || seqs[k] >= B->batch)
-            return vo_set_err(ctx, B200VO_E_BADARG, "seqs[%d] = %d is outside [0, batch = %d)", k, seqs[k], B->batch);
-        if (seen[seqs[k]]++) return vo_set_err(ctx, B200VO_E_BADARG, "sequence %d is listed twice", seqs[k]);
         // the slot bounds the frame; the window bounds it from below as it bounds cfg->rows / cfg->cols (and with it the
         // detector's 3 x 3 minimum)
         if (rows[k] > c.rows || cols[k] > c.cols)
@@ -216,70 +256,36 @@ int batch_set_frame_size(b200vo_batch* B, int n_seq, const int32_t* seqs, const 
             return vo_set_err(ctx, B200VO_E_BADARG, "sequence %d: %d x %d is not larger than the %d x %d window", seqs[k], rows[k], cols[k],
                               c.win_h, c.win_w);
     }
-    if (B->q_count > 0) return vo_set_err(ctx, B200VO_E_BADARG, "submitted frame sets are waiting: their pyramids were built at the old sizes");
-    std::vector<VoSeqExt> ext = B->ext_host;
-    for (int k = 0; k < n_seq; ++k) vo_seq_ext(rows[k], cols[k], c.win_w, c.win_h, c.max_level, &ext[seqs[k]]);
-    bool uniform = true;
-    for (const VoSeqExt& e : ext) uniform = uniform && e.w[0] == c.cols && e.h[0] == c.rows;
-    VO_CUDA(ctx, cudaSetDevice(ctx->device));
-    VO_CUDA(ctx, cudaStreamSynchronize(ctx->stream));   // no step in flight reads the rows
-    VO_CUDA(ctx, cudaStreamSynchronize(B->pre_stream));
-    VO_CUDA(ctx, cudaMemcpyAsync(B->ext_buf.p, ext.data(), ext.size() * sizeof(VoSeqExt), cudaMemcpyHostToDevice, ctx->stream));
-    VO_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    B->ext_host.swap(ext);
-    B->ext = uniform ? nullptr : (const VoSeqExt*)B->ext_buf.p;
-    // a mask has its sequence's frame size: the listed sequences lose theirs
-    bool had_mask = false;
-    for (int k = 0; k < n_seq; ++k) had_mask = had_mask || B->mask_host[seqs[k]];
-    if (had_mask) VO_TRY(batch_set_detection_mask(B, n_seq, seqs, nullptr));
-    // a map covers its sequence's frame size: the listed sequences with distortion keep their coefficients, with new maps
-    VO_TRY(batch_build_maps(B, n_seq, seqs));
-    return 0;
+    std::vector<VoSeqSettings> next = B->seq;
+    for (int k = 0; k < n_seq; ++k) vo_seq_ext(rows[k], cols[k], c.win_w, c.win_h, c.max_level, &next[seqs[k]].ext);
+    return batch_apply(B, VO_SET_FRAME_SIZE, next, n_seq, seqs, nullptr, stale);
 }
 
-int batch_set_distortion(b200vo_batch* B, int n_seq, const int32_t* seqs, const double* dist)
+int batch_set_distortion(b200vo_batch* B, int n_seq, const int32_t* seqs, const double* dist, bool* stale)
 {
     b200vo_ctx* ctx = B->ctx;
-    const b200vo_batch_cfg& c = B->cfg;
-    if (n_seq < 1 || n_seq > B->batch) return vo_set_err(ctx, B200VO_E_BADARG, "n_seq = %d is outside [1, batch = %d]", n_seq, B->batch);
-    if (!seqs || !dist) return vo_set_err(ctx, B200VO_E_BADARG, "null array");
-    std::vector<char> seen(B->batch, 0);
-    for (int k = 0; k < n_seq; ++k) {
-        if (seqs[k] < 0 || seqs[k] >= B->batch)
-            return vo_set_err(ctx, B200VO_E_BADARG, "seqs[%d] = %d is outside [0, batch = %d)", k, seqs[k], B->batch);
-        if (seen[seqs[k]]++) return vo_set_err(ctx, B200VO_E_BADARG, "sequence %d is listed twice", seqs[k]);
+    VO_TRY(vo_check_seqs(ctx, B->batch, n_seq, seqs));
+    if (!dist) return vo_set_err(ctx, B200VO_E_BADARG, "null array");
+    for (int k = 0; k < n_seq; ++k)
         if (!vo_dist_valid(dist + 8 * (size_t)k)) return vo_set_err(ctx, B200VO_E_BADARG, "sequence %d: non-finite distortion coefficient", seqs[k]);
-    }
-    if (B->q_count > 0) return vo_set_err(ctx, B200VO_E_BADARG, "submitted frame sets are waiting: their pyramids were built with the old maps");
-    std::vector<double> coef = B->dist_host;
-    std::vector<uint8_t> on = B->dist_on;
-    bool any_new = false;
-    for (int k = 0; k < n_seq; ++k) {
-        bool nz = false;
-        for (int i = 0; i < 8; ++i) nz = nz || dist[8 * (size_t)k + i] != 0.0;
-        for (int i = 0; i < 8; ++i) coef[8 * (size_t)seqs[k] + i] = nz ? dist[8 * (size_t)k + i] : 0.0;
-        on[seqs[k]] = nz ? 1 : 0;
-        any_new = any_new || nz;
-    }
-    const size_t fb = (size_t)c.rows * c.cols, b_on = vo_align((size_t)B->batch, 256);
-    VO_CUDA(ctx, cudaSetDevice(ctx->device));
-    VO_CUDA(ctx, cudaStreamSynchronize(ctx->stream));   // no step in flight reads the maps
-    VO_CUDA(ctx, cudaStreamSynchronize(B->pre_stream));
-    if (any_new) VO_TRY(vo_reserve(ctx, B->dist_buf, b_on + B->batch * fb * 6));
-    B->dist_host.swap(coef);
-    B->dist_on.swap(on);
-    if (B->dist_buf.p) {
-        VO_CUDA(ctx, cudaMemcpyAsync(B->dist_buf.p, B->dist_on.data(), B->dist_on.size(), cudaMemcpyHostToDevice, ctx->stream));
-        VO_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    }
-    return batch_build_maps(B, n_seq, seqs);
+    std::vector<VoSeqSettings> next = B->seq;
+    for (int k = 0; k < n_seq; ++k) memcpy(next[seqs[k]].dist, dist + 8 * (size_t)k, 8 * sizeof(double));
+    return batch_apply(B, VO_SET_DISTORTION, next, n_seq, seqs, nullptr, stale);
+}
+
+int batch_set_detection_mask(b200vo_batch* B, int n_seq, const int32_t* seqs, const uint8_t* masks, bool* stale)
+{
+    VO_TRY(vo_check_seqs(B->ctx, B->batch, n_seq, seqs));
+    std::vector<VoSeqSettings> next = B->seq;
+    for (int k = 0; k < n_seq; ++k) next[seqs[k]].mask = masks != nullptr;
+    return batch_apply(B, VO_SET_MASK, next, n_seq, seqs, masks, stale);
 }
 
 VoUndist batch_undist(const b200vo_batch* B, int b0, int n, const int32_t* list)
 {
     VoUndist u;
     bool any = false;
-    for (int k = 0; k < n; ++k) any = any || B->dist_on[list ? list[k] : b0 + k];
+    for (int k = 0; B->n_dist && !any && k < n; ++k) any = B->seq[list ? list[k] : b0 + k].distorted();
     if (!any) return u;
     const size_t fb = (size_t)B->cfg.rows * B->cfg.cols;
     const uint8_t* d = (const uint8_t*)B->dist_buf.p;
@@ -292,51 +298,10 @@ VoUndist batch_undist(const b200vo_batch* B, int b0, int n, const int32_t* list)
     return u;
 }
 
-extern "C" int b200vo_batch_set_distortion(b200vo_batch* B, int n_seq, const int32_t* seqs, const double* dist)
-{
-    if (!B) return B200VO_E_BADARG;
-    VO_TRY(batch_set_distortion(B, n_seq, seqs, dist));
-    B->primed = false;   // the resident pyramids were built with the old maps
-    return 0;
-}
-
-int batch_set_detection_mask(b200vo_batch* B, int n_seq, const int32_t* seqs, const uint8_t* masks)
-{
-    b200vo_ctx* ctx = B->ctx;
-    const b200vo_batch_cfg& c = B->cfg;
-    if (n_seq < 1 || n_seq > B->batch) return vo_set_err(ctx, B200VO_E_BADARG, "n_seq = %d is outside [1, batch = %d]", n_seq, B->batch);
-    if (!seqs) return vo_set_err(ctx, B200VO_E_BADARG, "null array");
-    std::vector<char> seen(B->batch, 0);
-    for (int k = 0; k < n_seq; ++k) {
-        if (seqs[k] < 0 || seqs[k] >= B->batch)
-            return vo_set_err(ctx, B200VO_E_BADARG, "seqs[%d] = %d is outside [0, batch = %d)", k, seqs[k], B->batch);
-        if (seen[seqs[k]]++) return vo_set_err(ctx, B200VO_E_BADARG, "sequence %d is listed twice", seqs[k]);
-    }
-    const size_t fb = (size_t)c.rows * c.cols, b_on = vo_align((size_t)B->batch, 256);
-    std::vector<uint8_t> on = B->mask_host;
-    for (int k = 0; k < n_seq; ++k) on[seqs[k]] = masks ? 1 : 0;
-    VO_CUDA(ctx, cudaSetDevice(ctx->device));
-    VO_CUDA(ctx, cudaStreamSynchronize(ctx->stream));   // no step in flight reads the masks
-    VO_CUDA(ctx, cudaStreamSynchronize(B->pre_stream));
-    if (masks) VO_TRY(vo_reserve(ctx, B->mask_buf, b_on + B->batch * fb));
-    if (B->mask_buf.p) {
-        uint8_t* d = (uint8_t*)B->mask_buf.p;
-        if (masks)
-            for (int k = 0; k < n_seq; ++k)
-                VO_CUDA(ctx, cudaMemcpyAsync(d + b_on + seqs[k] * fb, masks + k * fb, fb, cudaMemcpyHostToDevice, ctx->stream));
-        VO_CUDA(ctx, cudaMemcpyAsync(d, on.data(), on.size(), cudaMemcpyHostToDevice, ctx->stream));
-        VO_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    }
-    B->mask_host.swap(on);
-    return 0;
-}
-
 VoMask batch_mask(const b200vo_batch* B)
 {
     VoMask m;
-    bool any = false;
-    for (uint8_t f : B->mask_host) any = any || f;
-    if (!any) return m;
+    if (!B->n_mask) return m;
     const uint8_t* d = (const uint8_t*)B->mask_buf.p;
     m.on = d;
     m.px = d + vo_align((size_t)B->batch, 256);
@@ -345,17 +310,47 @@ VoMask batch_mask(const b200vo_batch* B)
     return m;
 }
 
-extern "C" int b200vo_batch_set_detection_mask(b200vo_batch* B, int n_seq, const int32_t* seqs, const uint8_t* masks)
+int batch_pyramids(b200vo_batch* B, const uint8_t* raw, int set, int b0, int n, cudaStream_t stream, const int* list_dev,
+                   const int32_t* list_host)
 {
-    return B ? batch_set_detection_mask(B, n_seq, seqs, masks) : B200VO_E_BADARG;
+    const b200vo_batch_cfg& c = B->cfg;
+    const size_t sb = B->geom.slab_bytes;
+    return vo_build_pyramids(B->ctx, raw, (size_t)c.rows * c.cols, c.rows, c.cols, B->geom, (uint8_t*)B->slabs[set].p + (size_t)b0 * sb, sb,
+                             n, stream, B->ext ? B->ext + b0 : nullptr, B->ext ? &B->seq[b0].ext : nullptr, sizeof(VoSeqSettings), 0,
+                             list_dev, list_host, list_dev ? B->batch : 0, batch_undist(B, b0, n, list_host));
+}
+
+// The C setters: a setting that leaves the resident pyramids stale leaves the batch to be primed again
+extern "C" int b200vo_batch_set_intrinsics(b200vo_batch* B, int n_seq, const int32_t* seqs, const double* K)
+{
+    bool stale = false;
+    const int rc = B ? batch_set_intrinsics(B, n_seq, seqs, K, &stale) : B200VO_E_BADARG;
+    if (stale) B->primed = false;
+    return rc;
 }
 
 extern "C" int b200vo_batch_set_frame_size(b200vo_batch* B, int n_seq, const int32_t* seqs, const int32_t* rows, const int32_t* cols)
 {
-    if (!B) return B200VO_E_BADARG;
-    VO_TRY(batch_set_frame_size(B, n_seq, seqs, rows, cols));
-    B->primed = false;   // the resident pyramids were built at the old sizes
-    return 0;
+    bool stale = false;
+    const int rc = B ? batch_set_frame_size(B, n_seq, seqs, rows, cols, &stale) : B200VO_E_BADARG;
+    if (stale) B->primed = false;
+    return rc;
+}
+
+extern "C" int b200vo_batch_set_distortion(b200vo_batch* B, int n_seq, const int32_t* seqs, const double* dist)
+{
+    bool stale = false;
+    const int rc = B ? batch_set_distortion(B, n_seq, seqs, dist, &stale) : B200VO_E_BADARG;
+    if (stale) B->primed = false;
+    return rc;
+}
+
+extern "C" int b200vo_batch_set_detection_mask(b200vo_batch* B, int n_seq, const int32_t* seqs, const uint8_t* masks)
+{
+    bool stale = false;
+    const int rc = B ? batch_set_detection_mask(B, n_seq, seqs, masks, &stale) : B200VO_E_BADARG;
+    if (stale) B->primed = false;
+    return rc;
 }
 
 __global__ void trace_stamp_kernel(unsigned long long* dst)
@@ -448,9 +443,7 @@ static int batch_upload_frames(b200vo_batch* B, const uint8_t* frames, int slab_
         src = (const uint8_t*)ctx->h_pin;
     }
     VO_CUDA(ctx, cudaMemcpyAsync(B->raw.p, src, total, cudaMemcpyHostToDevice, ctx->stream));
-    VO_TRY(vo_build_pyramids(ctx, (const uint8_t*)B->raw.p, fb, B->cfg.rows, B->cfg.cols, B->geom,
-                             (uint8_t*)B->slabs[slab_set].p, B->geom.slab_bytes, B->batch, ctx->stream, batch_ext_dev(B, 0), batch_ext_host(B, 0),
-                             0, nullptr, nullptr, 0, batch_undist(B, 0, B->batch)));
+    VO_TRY(batch_pyramids(B, (const uint8_t*)B->raw.p, slab_set, 0, B->batch, ctx->stream));
     return 0;
 }
 
@@ -541,13 +534,9 @@ int batch_issue_prefetch(b200vo_batch* B, cudaEvent_t after, bool wait_step_end)
             raw = (const uint8_t*)B->raw_pre.p;
         }
         if (ql.empty())
-            VO_TRY(vo_build_pyramids(ctx, raw, fb, B->cfg.rows, B->cfg.cols, B->geom,
-                                     (uint8_t*)B->slabs[B->q_set[slot]].p, B->geom.slab_bytes, B->batch, B->pre_stream, batch_ext_dev(B, 0),
-                                     batch_ext_host(B, 0), 0, nullptr, nullptr, 0, batch_undist(B, 0, B->batch)));
+            VO_TRY(batch_pyramids(B, raw, B->q_set[slot], 0, B->batch, B->pre_stream));
         else
-            VO_TRY(vo_build_pyramids(ctx, raw, fb, B->cfg.rows, B->cfg.cols, B->geom, (uint8_t*)B->slabs[B->q_set[slot]].p,
-                                     B->geom.slab_bytes, (int)ql.size(), B->pre_stream, batch_ext_dev(B, 0), batch_ext_host(B, 0), 0,
-                                     batch_list_row(B, slot), ql.data(), B->batch, batch_undist(B, 0, (int)ql.size(), ql.data())));
+            VO_TRY(batch_pyramids(B, raw, B->q_set[slot], 0, (int)ql.size(), B->pre_stream, batch_list_row(B, slot), ql.data()));
         VO_CUDA(ctx, cudaEventRecord(B->q_ev[slot], B->pre_stream));
         B->q_src[slot] = nullptr;
     }
@@ -586,13 +575,9 @@ static int batch_track(b200vo_batch* B, cudaStream_t stream, int b0, int nb, con
         const bool whole = b0 == 0 && nb == B->batch;   // chunked uploads build the pyramids piecewise: no single interval to time
         if (whole) prof_mark(B, 0, stream);
         if (frames_dev && B->step_list)   // the listed images into their sequences' slabs (b0 == 0, nb == batch)
-            VO_TRY(vo_build_pyramids(ctx, frames_dev, fb, c.rows, c.cols, B->geom, (uint8_t*)B->slabs[nxt].p, sb, B->step_n, stream,
-                                     batch_ext_dev(B, 0), batch_ext_host(B, 0), 0, B->step_list, B->step_list_host, B->batch,
-                                     batch_undist(B, 0, B->step_n, B->step_list_host)));
+            VO_TRY(batch_pyramids(B, frames_dev, nxt, 0, B->step_n, stream, B->step_list, B->step_list_host));
         else if (frames_dev)
-            VO_TRY(vo_build_pyramids(ctx, frames_dev + (size_t)b0 * fb, fb, c.rows, c.cols, B->geom,
-                                     (uint8_t*)B->slabs[nxt].p + (size_t)b0 * sb, sb, nb, stream, batch_ext_dev(B, b0), batch_ext_host(B, b0),
-                                     0, nullptr, nullptr, 0, batch_undist(B, b0, nb)));
+            VO_TRY(batch_pyramids(B, frames_dev + (size_t)b0 * fb, nxt, b0, nb, stream));
         if (whole) { prof_mark(B, 1, stream); B->prof_row_open = B->profile && B->prof_n < B200VO_PROF_RING; }
     }
     KltPointSet sets[2] = {{L, n_lm + b0, lm_pts + (size_t)b0 * L * 2, lm_next + (size_t)b0 * L * 2, lm_status + (size_t)b0 * L, nullptr},
@@ -602,7 +587,7 @@ static int batch_track(b200vo_batch* B, cudaStream_t stream, int b0, int nb, con
     const KltPointSet* first = which == 2 ? sets + 1 : sets;
     const int n_sets = which == 0 ? (Cn > 0 ? 2 : 1) : 1;   // which 1, 4: landmark set; 2: candidate set
     VO_TRY(vo_klt_launch2(ctx, B->geom, (const uint8_t*)B->slabs[B->cur].p + (size_t)b0 * sb, sb,
-                          (const uint8_t*)B->slabs[nxt].p + (size_t)b0 * sb, sb, nb, first, n_sets, 0, B->kp, stream, batch_ext_dev(B, b0)));
+                          (const uint8_t*)B->slabs[nxt].p + (size_t)b0 * sb, sb, nb, first, n_sets, 0, B->kp, stream, B->ext ? B->ext + b0 : nullptr));
     return 0;
 }
 

@@ -9,6 +9,21 @@
 // host-buffer steps whose point arrays and results together stay below this go up / come back as ONE copy each
 #define B200VO_PACKED_IO_BYTES (512 * 1024)
 
+// One sequence's settings as the host keeps them (b200vo_batch_set_intrinsics / _frame_size / _detection_mask /
+// _distortion); the device holds their forms the kernels read (b200vo_batch::intr_buf, ext_buf, mask_buf, dist_buf)
+struct VoSeqSettings {
+    VoIntrinsics intr;
+    VoSeqExt ext;
+    double dist[8];   // k1, k2, p1, p2, k3, k4, k5, k6; all zero: no distortion
+    bool mask;        // has a detection mask
+    bool distorted() const
+    {
+        for (double d : dist)
+            if (d != 0.0) return true;
+        return false;
+    }
+};
+
 struct b200vo_batch {
     b200vo_ctx* ctx;
     int batch;
@@ -52,27 +67,22 @@ struct b200vo_batch {
     void* pnp_ws;
     const uint32_t* rng; int n_raw;
     bool primed;
-    // the camera of every sequence (b200vo_batch_set_intrinsics): device rows read by the kernels, host mirror of them
+    // the settings of every sequence (batch_apply): the host table, how many sequences have a mask / distortion, and the
+    // device forms.  intr_buf: the VoIntrinsics rows.  ext_buf: the VoSeqExt rows, read by the pyramid, tracker and detector
+    // kernels; `ext` is nullptr while every sequence has the slot size cfg.rows x cfg.cols: the kernels then take the slot
+    // geometry from their launch arguments, as a batch without per-sequence sizes always did.  mask_buf: [batch] "has a
+    // mask" bytes, then [batch] masks in the slot layout, allocated with the first mask.  dist_buf: [batch] "has distortion"
+    // bytes, then [batch] int16 source-pixel maps and [batch] uint16 fraction maps in the slot layout (VoUndist), allocated
+    // with the first distortion.  n_mask == 0: the detectors get no mask; n_dist == 0: pyramids as without distortion.
+    std::vector<VoSeqSettings> seq;
+    int n_mask = 0, n_dist = 0;
     DevBuf intr_buf;
     const VoIntrinsics* intr = nullptr;
-    std::vector<VoIntrinsics> intr_host;
-    // the frame size of every sequence (b200vo_batch_set_frame_size): device rows read by the pyramid, tracker and detector
-    // kernels, host mirror of them.  `ext` is nullptr while every sequence has the slot size cfg.rows x cfg.cols: the
-    // kernels then take the slot geometry from their launch arguments, as a batch without per-sequence sizes always did.
     DevBuf ext_buf;
     const VoSeqExt* ext = nullptr;
-    std::vector<VoSeqExt> ext_host;
-    // the detection mask of every sequence (b200vo_batch_set_detection_mask): [batch] "has a mask" bytes, then [batch] masks
-    // in the slot layout, allocated with the first mask.  mask_host mirrors the flags; no flag set: the detectors get no mask.
     DevBuf mask_buf;
-    std::vector<uint8_t> mask_host;
-    // the lens distortion of every sequence (b200vo_batch_set_distortion): [batch] "has distortion" bytes, then [batch]
-    // int16 source-pixel maps and [batch] uint16 fraction maps in the slot layout (VoUndist), allocated with the first
-    // distortion.  dist_host: the coefficients, [batch][8]; dist_on mirrors the flags; no flag set: pyramids as without.
     DevBuf dist_buf;
     DevBuf dist_par;                // the parameter rows of the last map build
-    std::vector<double> dist_host;
-    std::vector<uint8_t> dist_on;
     // host-input path: frames arrive chunk by chunk on a copy stream while earlier chunks are tracked
     cudaStream_t chunk_stream[B200VO_BATCH_STREAMS] = {};  // chunk k: H2D -> pyramid -> KLT on stream k % STREAMS
     cudaEvent_t chunk_ev[B200VO_BATCH_CHUNKS] = {};
@@ -107,22 +117,20 @@ int batch_track_pose_overlapped(b200vo_batch* B, const uint8_t* frames_dev, cons
                                 uint8_t* pnp_ok, uint8_t* inlier_mask, int* n_inliers, cudaEvent_t obj_ready,
                                 cudaEvent_t cand_ready = nullptr);
 int batch_finish(b200vo_batch* B);
-// Validates the (index, K) pairs and, only when all are valid, waits for the work in flight and uploads the new rows (synchronous)
-int batch_set_intrinsics(b200vo_batch* B, int n_seq, const int32_t* seqs, const double* K);
-// Validates the (index, rows, cols) triples and, only when all are valid and no submitted frame set waits, waits for the
-// work in flight and uploads the new extents (synchronous)
-int batch_set_frame_size(b200vo_batch* B, int n_seq, const int32_t* seqs, const int32_t* rows, const int32_t* cols);
-// Validates the n_seq distinct indices and, only when all are valid, waits for the work in flight and uploads the listed
-// sequences' masks (uint8 [n_seq][cfg.rows][cfg.cols]), or clears them (masks == nullptr).  Synchronous.
-int batch_set_detection_mask(b200vo_batch* B, int n_seq, const int32_t* seqs, const uint8_t* masks);
+// The setters of the listed sequences' settings: each checks its inputs and, only when all are valid and no submitted frame
+// set that depends on the setting waits, waits for the work in flight and applies the new rows (synchronous).  *stale:
+// the listed sequences' resident pyramids no longer match their frames (new sizes or maps).
+int batch_set_intrinsics(b200vo_batch* B, int n_seq, const int32_t* seqs, const double* K, bool* stale);
+int batch_set_frame_size(b200vo_batch* B, int n_seq, const int32_t* seqs, const int32_t* rows, const int32_t* cols, bool* stale);
+// masks: uint8 [n_seq][cfg.rows][cfg.cols], nullptr: the listed sequences' masks are cleared
+int batch_set_detection_mask(b200vo_batch* B, int n_seq, const int32_t* seqs, const uint8_t* masks, bool* stale);
+// dist: [n_seq][8] k1, k2, p1, p2, k3, k4, k5, k6; an all-zero row clears a sequence's distortion
+int batch_set_distortion(b200vo_batch* B, int n_seq, const int32_t* seqs, const double* dist, bool* stale);
 // the masks of the detectors: indexed by sequence, none while no sequence has one
 VoMask batch_mask(const b200vo_batch* B);
-// Validates the n_seq distinct indices and their coefficients (dist: [n_seq][8] k1, k2, p1, p2, k3, k4, k5, k6; an
-// all-zero row clears a sequence's distortion) and, only when all are valid and no submitted frame set waits, waits for
-// the work in flight and builds the listed sequences' maps.  Synchronous.
-int batch_set_distortion(b200vo_batch* B, int n_seq, const int32_t* seqs, const double* dist);
 // the maps of sequences b0 .. b0 + n - 1, or of the n sequences list[k] (b0 == 0); none while none of them has distortion
 VoUndist batch_undist(const b200vo_batch* B, int b0, int n, const int32_t* list = nullptr);
-// the device rows of sequences [b0, ...) and their host copy, or nullptr for both while every sequence has the slot size
-inline const VoSeqExt* batch_ext_dev(const b200vo_batch* B, int b0) { return B->ext ? B->ext + b0 : nullptr; }
-inline const VoSeqExt* batch_ext_host(const b200vo_batch* B, int b0) { return B->ext ? B->ext_host.data() + b0 : nullptr; }
+// The pyramids of n raw images (device, slot layout, one slot apart) into slab set `set`, each at its sequence's extents
+// and with its map: image k is sequence b0 + k, or with a list (its device row and host copy, b0 == 0) sequence list[k]
+int batch_pyramids(b200vo_batch* B, const uint8_t* raw, int set, int b0, int n, cudaStream_t stream, const int* list_dev = nullptr,
+                   const int32_t* list_host = nullptr);

@@ -82,21 +82,16 @@ int vo_intrinsics_uniform(b200vo_ctx* ctx, const double K[9], double emat_thr, i
     return 0;
 }
 
-int vo_intrinsics_set(b200vo_ctx* ctx, int batch, int n_seq, const int32_t* seqs, const double* K, double emat_thr,
-                      VoIntrinsics* rows)
+int vo_check_seqs(b200vo_ctx* ctx, int batch, int n_seq, const int32_t* seqs)
 {
     if (n_seq < 1 || n_seq > batch) return vo_set_err(ctx, B200VO_E_BADARG, "n_seq = %d is outside [1, batch = %d]", n_seq, batch);
-    if (!seqs || !K) return vo_set_err(ctx, B200VO_E_BADARG, "null array");
+    if (!seqs) return vo_set_err(ctx, B200VO_E_BADARG, "null array");
     std::vector<char> seen(batch, 0);
     for (int k = 0; k < n_seq; ++k) {
         if (seqs[k] < 0 || seqs[k] >= batch)
             return vo_set_err(ctx, B200VO_E_BADARG, "seqs[%d] = %d is outside [0, batch = %d)", k, seqs[k], batch);
         if (seen[seqs[k]]++) return vo_set_err(ctx, B200VO_E_BADARG, "sequence %d is listed twice", seqs[k]);
-        if (!vo_intrinsics_valid(K + 9 * k))
-            return vo_set_err(ctx, B200VO_E_BADARG, "K[%d] is not a camera matrix: fx, fy finite and > 0, cx, cy finite, "
-                                                    "skew 0, last row (0, 0, 1)", k);
     }
-    for (int k = 0; k < n_seq; ++k) vo_intrinsics_row(rows[seqs[k]], K + 9 * k, emat_thr);
     return 0;
 }
 

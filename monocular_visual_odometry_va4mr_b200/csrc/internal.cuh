@@ -114,10 +114,6 @@ void vo_intrinsics_row(VoIntrinsics& r, const double K[9], double emat_thr);
 // The single-K entry points: n identical rows of K in the ctx's own buffer, uploaded on the ctx stream (pageable source,
 // staged before the call returns, so the upload never waits for the device)
 int vo_intrinsics_uniform(b200vo_ctx* ctx, const double K[9], double emat_thr, int n, const VoIntrinsics** d_rows);
-// Validates the n_seq (index, K) pairs of a set_intrinsics call against [0, batch) and fills rows[seqs[k]] of the host mirror
-// `rows` ([batch]); nothing is written unless every pair is valid
-int vo_intrinsics_set(b200vo_ctx* ctx, int batch, int n_seq, const int32_t* seqs, const double* K, double emat_thr,
-                      VoIntrinsics* rows);
 
 struct b200vo_ctx {
     int device = 0;
@@ -152,6 +148,8 @@ int vo_set_err(b200vo_ctx* ctx, int code, const char* fmt, ...);
 int vo_cuda_fail(b200vo_ctx* ctx, cudaError_t e, const char* what);
 int vo_reserve(b200vo_ctx* ctx, DevBuf& b, size_t bytes);
 int vo_reserve_pinned(b200vo_ctx* ctx, size_t bytes);
+// The list argument of the per-sequence calls: n_seq in [1, batch] distinct indices in [0, batch); B200VO_E_BADARG otherwise
+int vo_check_seqs(b200vo_ctx* ctx, int batch, int n_seq, const int32_t* seqs);
 
 #define VO_CUDA(ctx, call)                                         \
     do {                                                           \
@@ -209,12 +207,13 @@ void vo_seq_ext(int rows, int cols, int win_w, int win_h, int max_level, VoSeqEx
 // raw (device, rows of `raw_row` bytes, 0: cols) -> bordered level 0, then levels 1..L-1; `batch` slabs/raws strided.
 // d_ext / h_ext: [batch] per-sequence extents on the device and their host copy (both or neither), each inside the
 // slot geometry g; every level of a sequence is built at its own size, levels beyond its own count are not built.
+// h_ext_step: the bytes from one host row to the next (the rows may be members of larger per-sequence records).
 // d_list / h_list (both or neither): raw image k goes to slab list[k] of the n_slab slabs at d_slab, with the extents
 // ext[list[k]] (the tables then cover all n_slab slabs); the other slabs are not touched.
 // ud: the images' distortion maps, indexed like the extents (by slab); level 0 is then the undistorted image.
 int vo_build_pyramids(b200vo_ctx* ctx, const uint8_t* d_raw, size_t raw_stride, int rows, int cols,
                       const PyrGeom& g, uint8_t* d_slab, size_t slab_stride, int batch, cudaStream_t stream,
-                      const VoSeqExt* d_ext = nullptr, const VoSeqExt* h_ext = nullptr, size_t raw_row = 0,
+                      const VoSeqExt* d_ext = nullptr, const VoSeqExt* h_ext = nullptr, size_t h_ext_step = sizeof(VoSeqExt), size_t raw_row = 0,
                       const int* d_list = nullptr, const int* h_list = nullptr, int n_slab = 0, const VoUndist& ud = VoUndist{});
 
 // ---- undistort.cu ----

@@ -217,11 +217,9 @@ struct b200vo_loop {
     b200vo_loop_cfg cfg{};
     int batch = 0;
     DevBuf mem;                  // state + scratch
-    DevBuf res;                  // packed result block of b200vo_loop_step: pose_cw [batch][12] | status | n_inliers | n_lm | n_cand
-    size_t res_bytes = 0;
+    DevBuf res;                  // packed result block of the host steps: pose_cw [n][12] | status | n_inliers | n_lm | n_cand
     LoopDev d{};
     TriBatchArgs tri{};
-    LoopOut res_out{};
     DevBuf boot_in, boot_ws;     // b200vo_loop_bootstrap: frames and keypoint counts, everything after the matching
 };
 
@@ -259,8 +257,7 @@ extern "C" int b200vo_loop_create(b200vo_ctx* ctx, int batch, const b200vo_loop_
     size_t total = 0;
     for (size_t b : sizes) total += vo_align(b, 256);
     int rc = vo_reserve(ctx, lp->mem, total);
-    lp->res_bytes = nb * 96 + 4 * nb * 4;
-    if (!rc) rc = vo_reserve(ctx, lp->res, lp->res_bytes);
+    if (!rc) rc = vo_reserve(ctx, lp->res, nb * 96 + 4 * nb * 4);
     if (!rc) rc = vo_reserve(ctx, B->gftt_ws, vo_gftt_batch_workspace(bc.rows, bc.cols, batch, cfg->max_corners));
     if (!rc) rc = vo_reserve(ctx, B->lists, 3 * 2 * nb * sizeof(int32_t));
     if (rc) { b200vo_loop_destroy(lp); return rc; }
@@ -287,10 +284,6 @@ extern "C" int b200vo_loop_create(b200vo_ctx* ctx, int batch, const b200vo_loop_
     t.n = d.tri_n; t.n_poses = d.n_poses; t.cur = d.cur_pose;
     t.first_keys = d.fkeys_b; t.keys = d.keys_b; t.first_pose = d.fpose_b; t.poses = d.poses;
     t.keep = d.keep; t.lm_slot = lm_slot; t.out_lm = d.new_lm; t.out_kp = d.new_kp; t.n_new = d.n_new; t.flags = cnt + CNT_FLAGS * nb;
-    uint8_t* r = (uint8_t*)lp->res.p;
-    lp->res_out.pose = (double*)r;
-    lp->res_out.status = (int*)(r + nb * 96);
-    lp->res_out.n_inl = lp->res_out.status + nb; lp->res_out.n_lm = lp->res_out.n_inl + nb; lp->res_out.n_cand = lp->res_out.n_lm + nb;
     // every sequence starts IDLE with an empty state; the frames are blank until a sequence is loaded (the detector runs
     // over every image of the batch)
     std::vector<int> idle(batch, B200VO_LOOP_IDLE);
@@ -347,10 +340,12 @@ static int loop_core(b200vo_loop* lp, const uint8_t* frames_dev, const LoopOut& 
     return batch_finish(B);
 }
 
-// a full step must not consume a set that was submitted with a list
+// what a full step may consume: its own frames while no set waits, or the oldest submitted set if it has no list
 static int loop_check_full(b200vo_loop* lp, const uint8_t* frames)
 {
     const b200vo_batch* B = lp->B;
+    if (frames && B->q_count > 0)
+        return vo_set_err(lp->ctx, B200VO_E_BADARG, "submitted frame sets are waiting: pass frames == NULL to consume them in order");
     if (!frames && B->q_count > 0 && !B->q_list[B->q_head].empty())
         return vo_set_err(lp->ctx, B200VO_E_BADARG, "the oldest submitted frame set lists %d sequences: consume it with the listed step",
                           (int)B->q_list[B->q_head].size());
@@ -367,26 +362,27 @@ extern "C" int b200vo_loop_step_dev(b200vo_loop* lp, const uint8_t* frames_dev, 
     return loop_core(lp, frames_dev, o);
 }
 
-extern "C" int b200vo_loop_step(b200vo_loop* lp, const uint8_t* frames, int32_t* status, int32_t* n_inliers, int32_t* n_lm,
-                                int32_t* n_cand, double* pose_cw)
+// One host-buffer step of every sequence (list == nullptr) or of the n listed ones (checked): one upload of the frames,
+// one read-back of the result rows, packed as pose_cw [n][12] | status | n_inliers | n_lm | n_cand
+static int loop_step_host(b200vo_loop* lp, int n, const int32_t* list, const uint8_t* frames, int32_t* status, int32_t* n_inliers,
+                          int32_t* n_lm, int32_t* n_cand, double* pose_cw)
 {
-    if (!lp || !status || !n_inliers || !n_lm || !n_cand || !pose_cw) return B200VO_E_BADARG;
-    VO_TRY(loop_check_full(lp, frames));
     b200vo_ctx* ctx = lp->ctx;
     b200vo_batch* B = lp->B;
     VO_CUDA(ctx, cudaSetDevice(ctx->device));
     VO_CUDA(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
-    const size_t nb = lp->batch, f_total = (size_t)lp->cfg.batch.rows * lp->cfg.batch.cols * nb;
+    const size_t ns = n, f_total = (size_t)lp->cfg.batch.rows * lp->cfg.batch.cols * ns;
     bool pinned = false;
     if (frames) {
-        if (B->q_count > 0)
-            return vo_set_err(ctx, B200VO_E_BADARG, "submitted frame sets are waiting: pass frames == NULL to consume them in order");
         cudaPointerAttributes at{};
         pinned = cudaPointerGetAttributes(&at, frames) == cudaSuccess && at.type == cudaMemoryTypeHost;
         cudaGetLastError();
     }
+    uint8_t* r = (uint8_t*)lp->res.p;
+    const LoopOut o{(int*)(r + ns * 96), (int*)(r + ns * 96) + ns, (int*)(r + ns * 96) + 2 * ns, (int*)(r + ns * 96) + 3 * ns, (double*)r};
+    const size_t res_bytes = ns * 96 + 4 * ns * 4;
     const size_t staged = frames && !pinned ? vo_align(f_total, 256) : 0;
-    VO_TRY(vo_reserve_pinned(ctx, staged + lp->res_bytes));
+    VO_TRY(vo_reserve_pinned(ctx, staged + res_bytes));
     uint8_t* hp = (uint8_t*)ctx->h_pin;
     const uint8_t* fdev = nullptr;
     if (frames) {   // the one upload of the step
@@ -395,19 +391,27 @@ extern "C" int b200vo_loop_step(b200vo_loop* lp, const uint8_t* frames, int32_t*
         VO_CUDA(ctx, cudaMemcpyAsync(B->raw.p, pinned ? frames : hp, f_total, cudaMemcpyHostToDevice, ctx->stream));
         fdev = (const uint8_t*)B->raw.p;
     }
-    VO_TRY(loop_core(lp, fdev, lp->res_out));
+    VO_TRY(loop_core(lp, fdev, o, list ? n : 0, list));
     uint8_t* ho = hp + staged;   // the one read-back of the step
-    VO_CUDA(ctx, cudaMemcpyAsync(ho, lp->res.p, lp->res_bytes, cudaMemcpyDeviceToHost, ctx->stream));
+    VO_CUDA(ctx, cudaMemcpyAsync(ho, r, res_bytes, cudaMemcpyDeviceToHost, ctx->stream));
     VO_CUDA(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
     VO_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     cudaEventElapsedTime(&ctx->last_ms, ctx->ev0, ctx->ev1);
-    memcpy(pose_cw, ho, nb * 96);
-    const int* ri = (const int*)(ho + nb * 96);
-    memcpy(status, ri, nb * 4);
-    memcpy(n_inliers, ri + nb, nb * 4);
-    memcpy(n_lm, ri + 2 * nb, nb * 4);
-    memcpy(n_cand, ri + 3 * nb, nb * 4);
+    memcpy(pose_cw, ho, ns * 96);
+    const int* ri = (const int*)(ho + ns * 96);
+    memcpy(status, ri, ns * 4);
+    memcpy(n_inliers, ri + ns, ns * 4);
+    memcpy(n_lm, ri + 2 * ns, ns * 4);
+    memcpy(n_cand, ri + 3 * ns, ns * 4);
     return 0;
+}
+
+extern "C" int b200vo_loop_step(b200vo_loop* lp, const uint8_t* frames, int32_t* status, int32_t* n_inliers, int32_t* n_lm,
+                                int32_t* n_cand, double* pose_cw)
+{
+    if (!lp || !status || !n_inliers || !n_lm || !n_cand || !pose_cw) return B200VO_E_BADARG;
+    VO_TRY(loop_check_full(lp, frames));
+    return loop_step_host(lp, lp->batch, nullptr, frames, status, n_inliers, n_lm, n_cand, pose_cw);
 }
 
 extern "C" int b200vo_loop_submit_frames(b200vo_loop* lp, const uint8_t* frames)
@@ -423,27 +427,12 @@ extern "C" int b200vo_loop_submit_frames_dev(b200vo_loop* lp, const uint8_t* fra
 // ------------------------------------------------------------------------------------------
 // listed steps: only the sequences of a list advance
 // ------------------------------------------------------------------------------------------
-// n_seq distinct indices in [0, batch)
-static int loop_check_list(b200vo_loop* lp, int n_seq, const int32_t* seqs)
-{
-    b200vo_ctx* ctx = lp->ctx;
-    if (n_seq < 1 || n_seq > lp->batch) return vo_set_err(ctx, B200VO_E_BADARG, "n_seq = %d is outside [1, batch = %d]", n_seq, lp->batch);
-    if (!seqs) return vo_set_err(ctx, B200VO_E_BADARG, "null array");
-    std::vector<char> seen(lp->batch, 0);
-    for (int k = 0; k < n_seq; ++k) {
-        if (seqs[k] < 0 || seqs[k] >= lp->batch)
-            return vo_set_err(ctx, B200VO_E_BADARG, "seqs[%d] = %d is outside [0, batch = %d)", k, seqs[k], lp->batch);
-        if (seen[seqs[k]]++) return vo_set_err(ctx, B200VO_E_BADARG, "sequence %d is listed twice", seqs[k]);
-    }
-    return 0;
-}
-
 // what a listed step may consume: its own frames while no set waits, or the oldest submitted set if it has the same list
 static int loop_check_step_list(b200vo_loop* lp, int n_seq, const int32_t* seqs, const uint8_t* frames)
 {
     b200vo_ctx* ctx = lp->ctx;
     const b200vo_batch* B = lp->B;
-    VO_TRY(loop_check_list(lp, n_seq, seqs));
+    VO_TRY(vo_check_seqs(ctx, lp->batch, n_seq, seqs));
     if (frames) {
         if (B->q_count > 0)
             return vo_set_err(ctx, B200VO_E_BADARG, "submitted frame sets are waiting: pass frames == NULL to consume them in order");
@@ -472,59 +461,22 @@ extern "C" int b200vo_loop_step_seqs(b200vo_loop* lp, int n_seq, const int32_t* 
                                      int32_t* n_inliers, int32_t* n_lm, int32_t* n_cand, double* pose_cw)
 {
     if (!lp) return B200VO_E_BADARG;
-    b200vo_ctx* ctx = lp->ctx;
-    b200vo_batch* B = lp->B;
-    if (!status || !n_inliers || !n_lm || !n_cand || !pose_cw) return vo_set_err(ctx, B200VO_E_BADARG, "null array");
+    if (!status || !n_inliers || !n_lm || !n_cand || !pose_cw) return vo_set_err(lp->ctx, B200VO_E_BADARG, "null array");
     VO_TRY(loop_check_step_list(lp, n_seq, seqs, frames));
-    VO_CUDA(ctx, cudaSetDevice(ctx->device));
-    VO_CUDA(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
-    const size_t ns = n_seq, f_total = (size_t)lp->cfg.batch.rows * lp->cfg.batch.cols * ns;
-    bool pinned = false;
-    if (frames) {
-        cudaPointerAttributes at{};
-        pinned = cudaPointerGetAttributes(&at, frames) == cudaSuccess && at.type == cudaMemoryTypeHost;
-        cudaGetLastError();
-    }
-    // the result rows of the listed sequences, packed as the full step's block: pose_cw [n_seq][12] | status | n_inliers | n_lm | n_cand
-    uint8_t* r = (uint8_t*)lp->res.p;
-    const LoopOut o{(int*)(r + ns * 96), (int*)(r + ns * 96) + ns, (int*)(r + ns * 96) + 2 * ns, (int*)(r + ns * 96) + 3 * ns, (double*)r};
-    const size_t res_bytes = ns * 96 + 4 * ns * 4;
-    const size_t staged = frames && !pinned ? vo_align(f_total, 256) : 0;
-    VO_TRY(vo_reserve_pinned(ctx, staged + res_bytes));
-    uint8_t* hp = (uint8_t*)ctx->h_pin;
-    const uint8_t* fdev = nullptr;
-    if (frames) {   // the one upload of the step: the listed frames
-        VO_TRY(vo_reserve(ctx, B->raw, f_total));
-        if (!pinned) memcpy(hp, frames, f_total);
-        VO_CUDA(ctx, cudaMemcpyAsync(B->raw.p, pinned ? frames : hp, f_total, cudaMemcpyHostToDevice, ctx->stream));
-        fdev = (const uint8_t*)B->raw.p;
-    }
-    VO_TRY(loop_core(lp, fdev, o, n_seq, seqs));
-    uint8_t* ho = hp + staged;   // the one read-back of the step
-    VO_CUDA(ctx, cudaMemcpyAsync(ho, r, res_bytes, cudaMemcpyDeviceToHost, ctx->stream));
-    VO_CUDA(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
-    VO_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    cudaEventElapsedTime(&ctx->last_ms, ctx->ev0, ctx->ev1);
-    memcpy(pose_cw, ho, ns * 96);
-    const int* ri = (const int*)(ho + ns * 96);
-    memcpy(status, ri, ns * 4);
-    memcpy(n_inliers, ri + ns, ns * 4);
-    memcpy(n_lm, ri + 2 * ns, ns * 4);
-    memcpy(n_cand, ri + 3 * ns, ns * 4);
-    return 0;
+    return loop_step_host(lp, n_seq, seqs, frames, status, n_inliers, n_lm, n_cand, pose_cw);
 }
 
 extern "C" int b200vo_loop_submit_frames_seqs(b200vo_loop* lp, int n_seq, const int32_t* seqs, const uint8_t* frames)
 {
     if (!lp) return B200VO_E_BADARG;
-    VO_TRY(loop_check_list(lp, n_seq, seqs));
+    VO_TRY(vo_check_seqs(lp->ctx, lp->batch, n_seq, seqs));
     return batch_submit(lp->B, frames, false, n_seq, seqs);
 }
 
 extern "C" int b200vo_loop_submit_frames_seqs_dev(b200vo_loop* lp, int n_seq, const int32_t* seqs, const uint8_t* frames_dev)
 {
     if (!lp) return B200VO_E_BADARG;
-    VO_TRY(loop_check_list(lp, n_seq, seqs));
+    VO_TRY(vo_check_seqs(lp->ctx, lp->batch, n_seq, seqs));
     return batch_submit(lp->B, frames_dev, true, n_seq, seqs);
 }
 
@@ -549,14 +501,12 @@ extern "C" int b200vo_loop_load(b200vo_loop* lp, int seq, const uint8_t* frame, 
     VO_CUDA(ctx, cudaStreamSynchronize(ctx->stream));   // no step in flight reads the state
     cudaStream_t st = ctx->stream;
     const int rows = lp->cfg.batch.rows, cols = lp->cfg.batch.cols;
-    const size_t fb = (size_t)rows * cols, sb = B->geom.slab_bytes;
+    const size_t fb = (size_t)rows * cols;
     // the frame is tight at the sequence's own size: it becomes the top-left of a slot-layout frame
-    const int rs = B->ext_host[seq].h[0], cs = B->ext_host[seq].w[0];
+    const int rs = B->seq[seq].ext.h[0], cs = B->seq[seq].ext.w[0];
     VO_TRY(vo_reserve(ctx, B->raw, fb));
     VO_CUDA(ctx, cudaMemcpy2DAsync(B->raw.p, (size_t)cols, frame, (size_t)cs, (size_t)cs, (size_t)rs, cudaMemcpyHostToDevice, st));
-    VO_TRY(vo_build_pyramids(ctx, (const uint8_t*)B->raw.p, fb, rows, cols, B->geom,
-                             (uint8_t*)B->slabs[B->cur].p + (size_t)seq * sb, sb, 1, st, batch_ext_dev(B, seq), batch_ext_host(B, seq),
-                             0, nullptr, nullptr, 0, batch_undist(B, seq, 1)));
+    VO_TRY(batch_pyramids(B, (const uint8_t*)B->raw.p, B->cur, seq, 1, st));
     const size_t lo = (size_t)seq * d.L, co = (size_t)seq * d.C;
     if (n_lm > 0) {
         VO_CUDA(ctx, cudaMemcpyAsync(d.lm + 3 * lo, lm, (size_t)n_lm * 12, cudaMemcpyHostToDevice, st));
@@ -575,11 +525,6 @@ extern "C" int b200vo_loop_load(b200vo_loop* lp, int seq, const uint8_t* frame, 
     return 0;
 }
 
-extern "C" int b200vo_loop_set_intrinsics(b200vo_loop* lp, int n_seq, const int32_t* seqs, const double* K)
-{
-    return lp ? batch_set_intrinsics(lp->B, n_seq, seqs, K) : B200VO_E_BADARG;
-}
-
 // the listed sequences' pyramids no longer match their frames: IDLE (state arrays kept) until loaded or bootstrapped
 static int loop_idle(b200vo_loop* lp, int n_seq, const int32_t* seqs)
 {
@@ -595,23 +540,33 @@ static int loop_idle(b200vo_loop* lp, int n_seq, const int32_t* seqs)
     return 0;
 }
 
+// The C setters: a setting that leaves the listed sequences' resident pyramids stale makes them IDLE
+extern "C" int b200vo_loop_set_intrinsics(b200vo_loop* lp, int n_seq, const int32_t* seqs, const double* K)
+{
+    bool stale = false;
+    const int rc = lp ? batch_set_intrinsics(lp->B, n_seq, seqs, K, &stale) : B200VO_E_BADARG;
+    return stale ? loop_idle(lp, n_seq, seqs) : rc;
+}
+
 extern "C" int b200vo_loop_set_frame_size(b200vo_loop* lp, int n_seq, const int32_t* seqs, const int32_t* rows, const int32_t* cols)
 {
-    if (!lp) return B200VO_E_BADARG;
-    VO_TRY(batch_set_frame_size(lp->B, n_seq, seqs, rows, cols));
-    return loop_idle(lp, n_seq, seqs);
+    bool stale = false;
+    const int rc = lp ? batch_set_frame_size(lp->B, n_seq, seqs, rows, cols, &stale) : B200VO_E_BADARG;
+    return stale ? loop_idle(lp, n_seq, seqs) : rc;
 }
 
 extern "C" int b200vo_loop_set_distortion(b200vo_loop* lp, int n_seq, const int32_t* seqs, const double* dist)
 {
-    if (!lp) return B200VO_E_BADARG;
-    VO_TRY(batch_set_distortion(lp->B, n_seq, seqs, dist));
-    return loop_idle(lp, n_seq, seqs);
+    bool stale = false;
+    const int rc = lp ? batch_set_distortion(lp->B, n_seq, seqs, dist, &stale) : B200VO_E_BADARG;
+    return stale ? loop_idle(lp, n_seq, seqs) : rc;
 }
 
 extern "C" int b200vo_loop_set_detection_mask(b200vo_loop* lp, int n_seq, const int32_t* seqs, const uint8_t* masks)
 {
-    return lp ? batch_set_detection_mask(lp->B, n_seq, seqs, masks) : B200VO_E_BADARG;
+    bool stale = false;
+    const int rc = lp ? batch_set_detection_mask(lp->B, n_seq, seqs, masks, &stale) : B200VO_E_BADARG;
+    return stale ? loop_idle(lp, n_seq, seqs) : rc;
 }
 
 extern "C" int b200vo_loop_read_state(b200vo_loop* lp, int seq, float* lm, float* lm_kp, int32_t* n_lm, float* keys, float* first_keys,
@@ -763,14 +718,8 @@ extern "C" int b200vo_loop_bootstrap(b200vo_loop* lp, int n_seq, const int32_t* 
     if (!lp) return B200VO_E_BADARG;
     b200vo_ctx* ctx = lp->ctx;
     b200vo_batch* B = lp->B;
-    if (n_seq < 1 || n_seq > lp->batch) return vo_set_err(ctx, B200VO_E_BADARG, "n_seq = %d is outside [1, batch = %d]", n_seq, lp->batch);
-    if (!seqs || !frames0 || !frames1 || !status || !num_pts || !n_lm || !n_cand) return vo_set_err(ctx, B200VO_E_BADARG, "null array");
-    std::vector<char> seen(lp->batch, 0);
-    for (int k = 0; k < n_seq; ++k) {
-        if (seqs[k] < 0 || seqs[k] >= lp->batch)
-            return vo_set_err(ctx, B200VO_E_BADARG, "seqs[%d] = %d is outside [0, batch = %d)", k, seqs[k], lp->batch);
-        if (seen[seqs[k]]++) return vo_set_err(ctx, B200VO_E_BADARG, "sequence %d is listed twice", seqs[k]);
-    }
+    VO_TRY(vo_check_seqs(ctx, lp->batch, n_seq, seqs));
+    if (!frames0 || !frames1 || !status || !num_pts || !n_lm || !n_cand) return vo_set_err(ctx, B200VO_E_BADARG, "null array");
     const int rows = lp->cfg.batch.rows, cols = lp->cfg.batch.cols;
     const size_t fb = (size_t)rows * cols, sb = B->geom.slab_bytes, ns = n_seq;
     // The sequences run in groups of one frame size (SIFT works on one size per call), the groups in the order of their
@@ -781,9 +730,9 @@ extern "C" int b200vo_loop_bootstrap(b200vo_loop* lp, int n_seq, const int32_t* 
         std::vector<char> done(ns, 0);
         for (int k = 0; k < n_seq; ++k) {
             if (done[k]) continue;
-            const VoSeqExt& e = B->ext_host[seqs[k]];
+            const VoSeqExt& e = B->seq[seqs[k]].ext;
             for (int i = k; i < n_seq; ++i) {
-                const VoSeqExt& f = B->ext_host[seqs[i]];
+                const VoSeqExt& f = B->seq[seqs[i]].ext;
                 if (!done[i] && f.w[0] == e.w[0] && f.h[0] == e.h[0]) { done[i] = 1; perm.push_back(i); }
             }
             grp_end.push_back((int)perm.size());
@@ -813,7 +762,7 @@ extern "C" int b200vo_loop_bootstrap(b200vo_loop* lp, int n_seq, const int32_t* 
     long long* d_moff = nullptr;
     if (mk.px) {
         std::vector<long long> moff(2 * ns);
-        for (int j = 0; j < n_seq; ++j) moff[2 * j] = moff[2 * j + 1] = B->mask_host[seqs[j]] ? (long long)(seqs[j] * mk.stride) : -1;
+        for (int j = 0; j < n_seq; ++j) moff[2 * j] = moff[2 * j + 1] = B->seq[seqs[j]].mask ? (long long)(seqs[j] * mk.stride) : -1;
         d_moff = (long long*)(raw + b_raw + 2 * b_cnt);
         VO_CUDA(ctx, cudaMemcpyAsync(d_moff, moff.data(), ns * 16, cudaMemcpyHostToDevice, st));
     }
@@ -829,12 +778,12 @@ extern "C" int b200vo_loop_bootstrap(b200vo_loop* lp, int n_seq, const int32_t* 
     if (ud.xy) {   // frames 2j and 2j + 1 are sequence seqs[j]'s (run order)
         int* d_seq = (int*)(in + b_raw);
         VO_CUDA(ctx, cudaMemcpyAsync(d_seq, seqs, ns * 4, cudaMemcpyHostToDevice, st));
-        VO_TRY(vo_undistort_frames(ctx, in, raw, fb, (size_t)cols, 2 * n_seq, rows, cols, ud, d_seq, 1, batch_ext_dev(B, 0), st));
+        VO_TRY(vo_undistort_frames(ctx, in, raw, fb, (size_t)cols, 2 * n_seq, rows, cols, ud, d_seq, 1, B->ext, st));
     }
     // SIFT per size group, each group's keypoint and descriptor rows after the previous group's
     int n_rows = 0;
     for (size_t g = 0, j0 = 0; g < grp_end.size(); j0 = grp_end[g++]) {
-        const VoSeqExt& e = B->ext_host[seqs[j0]];
+        const VoSeqExt& e = B->seq[seqs[j0]].ext;
         const int m = grp_end[g] - (int)j0;
         VO_TRY(vo_sift_frames(ctx, raw + 2 * j0 * fb, fb, 2 * m, e.h[0], e.w[0], true, d_nkp + 2 * j0, d_row + 2 * j0, &n_rows, n_rows,
                               (size_t)cols, mk.px, d_moff ? d_moff + 2 * j0 : nullptr));
@@ -892,7 +841,7 @@ extern "C" int b200vo_loop_bootstrap(b200vo_loop* lp, int n_seq, const int32_t* 
     // the camera of each listed sequence, in list order (the bootstrap's kernels take the sequence from the grid)
     VoIntrinsics* intr = (VoIntrinsics*)take();
     std::vector<VoIntrinsics> h_intr(ns);
-    for (int k = 0; k < n_seq; ++k) h_intr[k] = B->intr_host[seqs[k]];
+    for (int k = 0; k < n_seq; ++k) h_intr[k] = B->seq[seqs[k]].intr;
     VO_CUDA(ctx, cudaMemcpyAsync(intr, h_intr.data(), ns * sizeof(VoIntrinsics), cudaMemcpyHostToDevice, st));
     t.intr = intr;
     b.keep = t.keep; b.new_lm = t.out_lm; b.new_kp = t.out_kp; b.n_new = t.n_new;
@@ -937,7 +886,7 @@ extern "C" int b200vo_loop_bootstrap(b200vo_loop* lp, int n_seq, const int32_t* 
     VO_TRY(vo_triangulate_batch_launch(ctx, t, n_seq, st));
     // the second frames' pyramids, each at its sequence's size (the run's own table; none while every size is the slot's)
     std::vector<VoSeqExt> h_ext(ns);
-    for (int j = 0; j < n_seq; ++j) h_ext[j] = B->ext_host[seqs[j]];
+    for (int j = 0; j < n_seq; ++j) h_ext[j] = B->seq[seqs[j]].ext;
     if (B->ext) VO_CUDA(ctx, cudaMemcpyAsync(ext_run, h_ext.data(), ns * sizeof(VoSeqExt), cudaMemcpyHostToDevice, st));
     VO_TRY(vo_build_pyramids(ctx, raw + fb, 2 * fb, rows, cols, B->geom, slab, sb, n_seq, st, B->ext ? ext_run : nullptr,
                              B->ext ? h_ext.data() : nullptr));

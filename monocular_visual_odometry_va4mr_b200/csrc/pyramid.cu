@@ -348,7 +348,7 @@ static int pyr_src_map(b200vo_ctx* ctx, CUtensorMap* map, uint8_t* d_slab, size_
 
 int vo_build_pyramids(b200vo_ctx* ctx, const uint8_t* d_raw, size_t raw_stride, int rows, int cols,
                       const PyrGeom& g, uint8_t* d_slab, size_t slab_stride, int batch, cudaStream_t stream,
-                      const VoSeqExt* d_ext, const VoSeqExt* h_ext, size_t raw_row, const int* d_list, const int* h_list, int n_slab,
+                      const VoSeqExt* d_ext, const VoSeqExt* h_ext, size_t h_ext_step, size_t raw_row, const int* d_list, const int* h_list, int n_slab,
                       const VoUndist& ud)
 {
     if (!raw_row) raw_row = (size_t)cols;
@@ -381,7 +381,7 @@ int vo_build_pyramids(b200vo_ctx* ctx, const uint8_t* d_raw, size_t raw_stride, 
                 if (h_ext) {   // the single-bounce test per sequence: a ring is left to the border kernel if any tile set could not write it
                     fused = true;
                     for (int b = 0; b < batch; ++b) {
-                        const VoSeqExt& e = h_ext[h_list ? h_list[b] : b];
+                        const VoSeqExt& e = *(const VoSeqExt*)((const char*)h_ext + (size_t)(h_list ? h_list[b] : b) * h_ext_step);
                         if (l < e.levels && !(e.w[l] >= VO_BORDER + 2 && e.h[l] >= VO_BORDER + 2)) fused = false;
                     }
                 }
