@@ -17,7 +17,11 @@ Round 3 (the batch kind: SequenceBatch with per-sequence frame sizes, compared p
 random slots up to 519 x 1299, 1-8 sequences of random and near-minimal sizes, the six windows, maxLevel 0..7, all three criteria
 types, zero or random padding, two tracker steps and one detection): FUZZ_KINDS=batch, seeds 41 and 42, 250 s each, run side by
 side on one B200 = 496 + 467 batches, 7 600 + 7 352 per-sequence tracker comparisons, 2 222 + 2 153 per-sequence detections:
-0 mismatches."""
+0 mismatches.
+Round 4 (the batch kind with a random distortion model or none and a random mask kind or none per sequence, compared with the
+oracle on the undistorted image and with mask_reference): FUZZ_KINDS=batch, seeds 51 and 52, 150 s each, run side by side on one
+B200 (1000 W power limit) = 275 + 287 batches, 4 374 + 4 258 per-sequence tracker comparisons, 1 279 + 1 266 per-sequence
+detections, 867 + 847 distorted and 910 + 911 masked sequences: 0 mismatches."""
 import os
 import sys
 import time
@@ -26,17 +30,38 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden"))
 import numpy as np  # noqa: E402
 
+import mask_reference as MR  # noqa: E402
 import oracle  # noqa: E402
+import undistort_reference as U  # noqa: E402
 from make_golden import make_emat_pair, make_pnp_case, sift_like  # noqa: E402
 from monocular_visual_odometry_va4mr_b200 import _lib, cv2_compat, hotpath, synth  # noqa: E402
 from monocular_visual_odometry_va4mr_b200.batch import SequenceBatch  # noqa: E402
 
 WINDOWS = [(15, 15), (21, 21), (9, 13), (31, 31), (5, 7), (21, 15)]
+DIST_MODELS = list(U.MODELS) + [None, None]          # a sequence's lens distortion, or none
+MASK_KINDS = [None, None, "hood", "blob", "band", "pixels", "zero"]
+
+
+def _mask(kind, r, c, rng):
+    """the in-frame bytes of a detection mask of the given kind at r x c"""
+    if kind == "hood":
+        return MR.hood_mask((r, c))
+    if kind == "blob":
+        return MR.blob_mask((r, c), seed=int(rng.integers(0, 1000)))
+    m = np.zeros((r, c), np.uint8)
+    if kind == "band":                                # across the detector's fused / unfused column w & ~31
+        x = c & ~31
+        m[:, max(x - 4, 0):x + 4] = 255
+    elif kind == "pixels":
+        m[rng.integers(0, r, 6), rng.integers(0, c, 6)] = int(rng.integers(1, 256))
+    return m
 
 
 def batch_case(rng, bad, stats):
-    """SequenceBatch with per-sequence frame sizes: a random slot, random sizes (near-minimal ones included), window,
-    maxLevel, criteria and padding; two tracker steps and one detection, each sequence against the oracle on its own image."""
+    """SequenceBatch with per-sequence frame sizes, distortion and masks: a random slot, random sizes (near-minimal ones
+    included), window, maxLevel, criteria and padding, a random distortion model or none per sequence (its camera the KITTI
+    one scaled to its size) and a random mask kind or none; two tracker steps and one detection, each sequence against the
+    oracle on its own undistorted image (mask_reference with its mask)."""
     win = WINDOWS[int(rng.integers(0, len(WINDOWS)))]
     slot = (int(rng.integers(win[1] + 1, 520)), int(rng.integers(win[0] + 1, 1300)))
     ml = int(rng.integers(0, 8))
@@ -55,11 +80,27 @@ def batch_case(rng, bad, stats):
         y0, x0 = int(rng.integers(0, slot[0] - r + 1)), int(rng.integers(0, slot[1] - c + 1))
         crops.append(np.ascontiguousarray(full[:, y0:y0 + r, x0:x0 + c]))
     random_pad = rng.random() < 0.5
+    # per sequence: a distortion model (the raw crop is what the camera gives; the oracle sees it undistorted) with the
+    # KITTI camera scaled to the sequence's size, and a detection mask
+    Ks = np.stack([U.scale_K(synth.K_KITTI, r, c, 376, 1241, tuple(rng.uniform(-0.5, 0.5, 2))) for r, c in sizes])
+    models = [DIST_MODELS[int(rng.integers(0, len(DIST_MODELS)))] for _ in range(b)]
+    und = [im if m is None else np.stack([U.undistort(f, K, U.MODELS[m]) for f in im]) for im, K, m in zip(crops, Ks, models)]
+    kinds = [MASK_KINDS[int(rng.integers(0, len(MASK_KINDS)))] for _ in range(b)]
+    masks = [None if kd is None else _mask(kd, r, c, rng) for kd, (r, c) in zip(kinds, sizes)]
+    masked = [k for k in range(b) if masks[k] is not None]
+    stats["batch_dist"] += sum(m is not None and any(U.MODELS[m]) for m in models)
+    stats["batch_masked"] += len(masked)
 
     def layout(f):
         out = rng.integers(0, 256, (b,) + slot, dtype=np.uint8) if random_pad else np.zeros((b,) + slot, np.uint8)
         for k, im in enumerate(crops):
             out[k, :im.shape[1], :im.shape[2]] = im[f]
+        return out
+
+    def mask_layout():
+        out = rng.integers(1, 256, (len(masked),) + slot, dtype=np.uint8) if random_pad else np.zeros((len(masked),) + slot, np.uint8)
+        for j, k in enumerate(masked):
+            out[j, :sizes[k][0], :sizes[k][1]] = masks[k]
         return out
 
     pts = []
@@ -81,8 +122,10 @@ def batch_case(rng, bad, stats):
     n_pts = np.int32([len(p) for p in pts])
     n_cand = np.int32([len(p) if rng.random() < 0.7 else 0 for p in pts])
     cand_of = [np.ascontiguousarray(cand[k, :n_cand[k]]) for k in range(b)]
-    sb = SequenceBatch(b, *slot, synth.K_KITTI, win=win, max_level=ml, criteria=crit, max_landmarks=max(L, 4), max_candidates=L,
-                       frame_size=sizes)
+    sb = SequenceBatch(b, *slot, Ks, win=win, max_level=ml, criteria=crit, max_landmarks=max(L, 4), max_candidates=L,
+                       frame_size=sizes, dist_coeffs=[U.dist8(None if m is None else U.MODELS[m]) for m in models])
+    if masked:
+        sb.set_detection_mask(masked, mask_layout())
     obj = np.zeros((b, max(L, 4), 3), np.float32)
     lm4 = np.zeros((b, max(L, 4), 2), np.float32)
     lm4[:, :L] = lm
@@ -94,11 +137,11 @@ def batch_case(rng, bad, stats):
                 for name, p in (("lm", pts[k]), ("cand", cand_of[k])):
                     if not len(p):
                         continue
-                    rp, rst, _ = oracle.calc_optical_flow_pyr_lk(crops[k][f - 1], crops[k][f], p, win, ml, crit)
+                    rp, rst, _ = oracle.calc_optical_flow_pyr_lk(und[k][f - 1], und[k][f], p, win, ml, crit)
                     st, nxt = out[name + "_status"][k, :len(p)], out[name + "_next"][k, :len(p)]
                     ok = rst.ravel() == 1
                     if not (np.array_equal(st, rst.ravel()) and np.array_equal(nxt[ok], rp[ok])):
-                        bad.append(("batch-klt", slot, (r, c), win, ml, crit, f, name, int((st != rst.ravel()).sum())))
+                        bad.append(("batch-klt", slot, (r, c), models[k], win, ml, crit, f, name, int((st != rst.ravel()).sum())))
                     stats["batch_klt"] += 1
         mc = int(rng.choice([1, 7, 50, 1400, 5000]))
         q = float(rng.choice([0.1, 0.03, 0.01, 0.3]))
@@ -113,10 +156,13 @@ def batch_case(rng, bad, stats):
                 raise
             return
         for k in range(b):
-            want = oracle.good_features_to_track(crops[k][2], mc, q, md)
+            if masks[k] is None:
+                want = oracle.good_features_to_track(und[k][2], mc, q, md)
+            else:
+                want = MR.good_features_to_track(und[k][2], mc, q, md, mask=masks[k])
             want = np.zeros((0, 2), np.float32) if want is None else want.reshape(-1, 2)
             if nc[k] != len(want) or not np.array_equal(corners[k, :nc[k]], want):
-                bad.append(("batch-gftt", slot, sizes[k], mc, q, md, int(nc[k]), len(want)))
+                bad.append(("batch-gftt", slot, sizes[k], models[k], kinds[k], mc, q, md, int(nc[k]), len(want)))
             stats["batch_gftt"] += 1
     finally:
         sb.close()
@@ -126,7 +172,8 @@ def main():
     budget = float(sys.argv[1]) if len(sys.argv) > 1 else 120.0
     rng = np.random.default_rng(int(os.environ.get("FUZZ_SEED", "1")))
     t_end = time.time() + budget
-    stats = dict(klt=0, gftt=0, knn=0, pnp=0, emat=0, rpose=0, mind=0, tri=0, sift=0, batch=0, batch_klt=0, batch_gftt=0)
+    stats = dict(klt=0, gftt=0, knn=0, pnp=0, emat=0, rpose=0, mind=0, tri=0, sift=0, batch=0, batch_klt=0, batch_gftt=0, batch_dist=0,
+                 batch_masked=0)
     bad = []
     # FUZZ_KINDS=batch: only the batch kind
     only_batch = os.environ.get("FUZZ_KINDS", "") == "batch"
