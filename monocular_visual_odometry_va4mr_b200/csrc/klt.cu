@@ -35,6 +35,7 @@ struct KltArgs {
     int win_w, win_h, max_count;
     double eps_sq;
     float min_eig_thr;
+    float min_eig_num;      // v3: minEig < min_eig_thr as a bound on minEig's numerator (min_eig_num_bound)
     float eps_lo, eps_hi;   // eps_sq * (1 -+ 1e-6) in float: outside this band the float test decides
     // shared-memory carve-up (bytes, per warp)
     int patch_stride, smem_patch, smem_der, smem_iwin, smem_di, smem_per_warp;
@@ -305,12 +306,14 @@ int vo_klt_launch2(b200vo_ctx* ctx, const PyrGeom& g, const uint8_t* d_prev_slab
     void (*kern)(const KltArgs) = d_ext ? klt_kernel<0, 0, true> : klt_kernel<0, 0, false>;
     bool staged = false;
     // the staged kernel (persistent warps + work queue) for the two window sizes it is built for; the queue counter is
-    // an int, so a launch of 2^30 features or more takes the generic kernel (same arithmetic, same results)
+    // an int, so a launch of 2^30 features or more takes the generic kernel (same arithmetic, same results), and so do
+    // frames of 2^22 pixels or more in a dimension (the staged kernel's floor is exact below that: floor_v3)
     const bool sized = (kp.win_w == 21 && kp.win_h == 21) || (kp.win_w == 15 && kp.win_h == 15);
     unsigned launch_grid = grid;
-    if (sized && total_warps < (1ll << 30)) {
+    if (sized && total_warps < (1ll << 30) && g.w[0] < (1 << 22) && g.h[0] < (1 << 22)) {
         int min_ctas;
         staged = true;
+        a.min_eig_num = min_eig_num_bound(kp.min_eig_thr, (float)(2 * kp.win_w * kp.win_h));
         // per-sequence extents: the instances that read them (a uniform batch keeps the ones that take the launch's geometry)
         if (kp.win_w == 21) {
             kern = d_ext ? klt_kernel_v3<21, 21, true> : klt_kernel_v3<21, 21, false>;

@@ -15,13 +15,15 @@
 //     converges, so a CTA slot is never held by the slowest of four features, and small shards (8 sequences
 //     per GPU in the strong-scaling run) are not tail-bound (profiles/r2a_klt_source_hot.txt);
 //   * iteration loop: the staged-window test and the image-range test are ONE unsigned compare per axis
-//     against bounds fixed at staging time; plain F2I.FLOOR instead of the guarded cvFloor (positions are
-//     finite inside the loop, the guard stays at the level entry); the two exact 64-bit warp sums take a
+//     against bounds fixed at staging time; floor and cvRound by magic-constant FADDs instead of F2I / I2F, the
+//     packed weights straight from their bit patterns (klt_v3_forms.cuh); the two exact 64-bit warp sums take a
 //     single-REDUX fast path when a per-level bound rules out an int32 overflow (ITER_SUM_FAST_MAX; the hi/lo
-//     split path is kept for the rest); packed weights by one IMAD each;
+//     split path is kept for the rest);
+//   * level setup: the minEig test is a compare of its numerator against a bound found on the host (no division);
 //   * Iwin and the final error pass are skipped when the point set has no error output.
 #pragma once
 #include <type_traits>
+#include "klt_v3_forms.cuh"
 
 // 16-bit weights x 8-bit pixels.  The weights are SIGNED halves: iw11 = 2^14 - iw00 - iw01 - iw10 is -1
 // when the three rounded weights add up to 2^14 + 1 (a fractional part of ~0 in x or y, about one
@@ -263,6 +265,9 @@ klt_kernel_v3(const KltArgs a)
             if (t >= C::NTASK) { ty[r] = 0; tx[r] = 0; }
         }
     }
+    // split layout: the live pixels of the lane's run as masks, the first WW - 8 (live in both runs of a live row) and
+    // the rest (live in a left run of a live row only)
+    const int mrow = tl[0] > 0 ? -1 : 0, mtail = tl[0] == 8 ? -1 : 0;
     // this lane's byte offsets inside the staged J window, pinned to registers
     int joffl[C::NROUND];
 #pragma unroll
@@ -317,13 +322,25 @@ klt_kernel_v3(const KltArgs a)
         else { nx = __fmul_rn(outx, 2.f); ny = __fmul_rn(outy, 2.f); }
         outx = nx; outy = ny;
         ppx = __fsub_rn(ppx, hwx); ppy = __fsub_rn(ppy, hwy);
-        const int ipx = floor_to_int(ppx), ipy = floor_to_int(ppy);
+        uint32_t bpx, bpy;
+        const float fpx = floor_v3(ppx, bpx), fpy = floor_v3(ppy, bpy);
+        const int ipx = floor_bits_to_int(bpx), ipy = floor_bits_to_int(bpy);
         if (ipx < -WW || ipx >= lw || ipy < -WH || ipy >= lh) {
             if (level == 0) { st = 0; e = 0.f; }
             continue;
         }
+        // wt = iw00 | iw01 << 16, wb = iw10 | iw11 << 16.  The layouts of more than two runs per row (21x21) take every
+        // template through the per-tap path, which wants the four weights as integers: there the packed form costs a
+        // spill at 80 registers, so they keep the shared helper (the same weights)
+        uint32_t wt, wb;
         int iw00, iw01, iw10, iw11;
-        bilinear_weights(__fsub_rn(ppx, (float)ipx), __fsub_rn(ppy, (float)ipy), iw00, iw01, iw10, iw11);
+        if (C::SPLIT) {
+            bilinear_weights_v3(__fsub_rn(ppx, fpx), __fsub_rn(ppy, fpy), wt, wb);
+            iw00 = (int)(wt & 0xFFFF); iw01 = (int)(wt >> 16); iw10 = (int)(wb & 0xFFFF); iw11 = (int)wb >> 16;
+        } else {
+            bilinear_weights(__fsub_rn(ppx, fpx), __fsub_rn(ppy, fpy), iw00, iw01, iw10, iw11);
+            wt = (uint32_t)(iw01 * 65536 + iw00); wb = (uint32_t)iw11 * 65536u + (uint32_t)iw10;
+        }
 
         // ---- staging pipeline (cp.async): this level's patch of I was prefetched during the previous
         // level; now start (1) the window of J around the initial position and (2) the NEXT level's
@@ -340,8 +357,12 @@ klt_kernel_v3(const KltArgs a)
         }
         const float jx0 = __fsub_rn(nx, hwx), jy0 = __fsub_rn(ny, hwy);
         // staged J window: valid (inx, iny) are xlo + [0, xspan] x ylo + [0, yspan] = inside the window AND inside the
-        // image range cv2 accepts; jbase = byte offset of (xlo, ylo) in the window.  Nothing staged: the test always fails.
-        int xlo = 0x40000001, ylo = 0x40000001, jbase = 0;   // odd, > 2^24: no float floors to it, so the test cannot pass by accident
+        // image range cv2 accepts, tested on floor_v3's bit patterns: xlob = V3_FLOOR_BITS + xlo (mod 2^32); jbase = byte
+        // offset of (xlo, ylo) in the window.  Nothing staged: the test always fails -- the sentinel is the pattern of
+        // -3.7e-32, and RD(x + 1.5 * 2^23) is +-0 or at least 0.5 in magnitude (x and 1.5 * 2^23 are multiples of 0.5
+        // wherever they can cancel)
+        uint32_t xlob = 0x8B400001u, ylob = 0x8B400001u;
+        int jbase = 0;
         unsigned xspan = 0, yspan = 0;
         auto stage_J = [&](int inx, int iny) {
             const int ry0 = iny - C::MARGIN;
@@ -349,13 +370,16 @@ klt_kernel_v3(const KltArgs a)
             const int m2 = (int)(reinterpret_cast<uintptr_t>(s0) & 7);
             const int rx0 = inx - C::MARGIN - m2;
             stage_rows_async8<C::JSLOT, C::JR>(jreg_s, s0 - m2, pitch, lane);
-            xlo = max(rx0, -WW); ylo = max(ry0, -WH);
+            const int xlo = max(rx0, -WW), ylo = max(ry0, -WH);
             const int xhi = min(rx0 + C::JS - WW - 2, lw - 1), yhi = min(ry0 + C::JR - WH - 2, lh - 1);
             xspan = (unsigned)(xhi - xlo); yspan = (unsigned)(yhi - ylo);     // the staging position itself is valid: spans >= 0
+            xlob = (uint32_t)xlo + V3_FLOOR_BITS; ylob = (uint32_t)ylo + V3_FLOOR_BITS;
             jbase = (ylo - ry0) * C::JS + (xlo - rx0);
         };
         {
-            const int inx = __float2int_rd(jx0), iny = __float2int_rd(jy0);
+            uint32_t bx, by;
+            floor_v3(jx0, bx); floor_v3(jy0, by);
+            const int inx = floor_bits_to_int(bx), iny = floor_bits_to_int(by);
             if (!(inx < -WW || inx >= lw || iny < -WH || iny >= lh)) stage_J(inx, iny);
             cp_async_commit();
         }
@@ -363,7 +387,9 @@ klt_kernel_v3(const KltArgs a)
         if (level > 0) {
             const int nl = level - 1;
             const float sc2 = __int_as_float((127 - nl) << 23);
-            const int qx = floor_to_int(__fsub_rn(__fmul_rn(px0, sc2), hwx)), qy = floor_to_int(__fsub_rn(__fmul_rn(py0, sc2), hwy));
+            uint32_t bx, by;
+            floor_v3(__fsub_rn(__fmul_rn(px0, sc2), hwx), bx); floor_v3(__fsub_rn(__fmul_rn(py0, sc2), hwy), by);
+            const int qx = floor_bits_to_int(bx), qy = floor_bits_to_int(by);
             if (!(qx < -WW || qx >= (EXT ? ext->w[nl] : a.w[nl]) || qy < -WH || qy >= (EXT ? ext->h[nl] : a.h[nl]))) {
                 const uint8_t* n0 = prev + a.off[nl] + (long long)(qy - 1) * a.pitch[nl] + (qx - 1);
                 const int m3 = (int)(reinterpret_cast<uintptr_t>(n0) & 7);
@@ -377,14 +403,19 @@ klt_kernel_v3(const KltArgs a)
         // patch pixel (x, y), x in [-1, WW+1], y in [-1, WH+1], lives at byte (y+1)*PS + mis + 1 + x
 
         // ---- template: dIx/dIy (registers), normal matrix, sum(Iwin*dI), Iwin (smem, only for the error) ----
-        const uint32_t wt = (uint32_t)(iw01 * 65536 + iw00), wb = (uint32_t)iw11 * 65536u + (uint32_t)iw10;
         int gxr[C::NROUND][8], gyr[C::NROUND][8];
         int sA11 = 0, sA12 = 0, sA22 = 0, c1 = 0, c2 = 0;
         auto accumulate = [&](int r, const int* ix, const int* iy, const int* Iv) {
 #pragma unroll
             for (int k = 0; k < 8; ++k) {
-                const bool livek = k < tl[r];
-                const int ixv = livek ? ix[k] : 0, iyv = livek ? iy[k] : 0;
+                int ixv, iyv;
+                if (C::SPLIT) {
+                    const int m = k < WW - 8 ? mrow : mtail;
+                    ixv = ix[k] & m; iyv = iy[k] & m;
+                } else {
+                    const bool livek = k < tl[r];
+                    ixv = livek ? ix[k] : 0; iyv = livek ? iy[k] : 0;
+                }
                 gxr[r][k] = ixv; gyr[r][k] = iyv;
                 sA11 += ixv * ixv; sA12 += ixv * iyv; sA22 += iyv * iyv;
                 c1 += Iv[k] * ixv; c2 += Iv[k] * iyv;
@@ -483,13 +514,12 @@ klt_kernel_v3(const KltArgs a)
         A11 = __fmul_rn(A11, FLT_SCALE); A12 = __fmul_rn(A12, FLT_SCALE); A22 = __fmul_rn(A22, FLT_SCALE);
         float D = __fsub_rn(__fmul_rn(A11, A22), __fmul_rn(A12, A12));
         const float dA = __fsub_rn(A11, A22);
-        const float minEig = __fdiv_rn(
-            __fsub_rn(__fadd_rn(A22, A11),
-                      __fsqrt_rn(__fadd_rn(__fmul_rn(dA, dA), __fmul_rn(__fmul_rn(4.f, A12), A12)))),
-            (float)(2 * WW * WH));
+        // minEig = num / (2 * WW * WH); minEig < min_eig_thr is num < min_eig_num (min_eig_num_bound)
+        const float num = __fsub_rn(__fadd_rn(A22, A11),
+                                    __fsqrt_rn(__fadd_rn(__fmul_rn(dA, dA), __fmul_rn(__fmul_rn(4.f, A12), A12))));
         // the prefetched patch becomes the current one at the next level, whatever happens below
         if (pf_next) { pb ^= 1; pf_level = level - 1; }
-        if (minEig < a.min_eig_thr || D < 1.192092896e-07f) {
+        if (num < a.min_eig_num || D < 1.192092896e-07f) {
             if (level == 0) st = 0;
             cp_async_wait_pending(level > 0 ? 1 : 0);   // drain the J window copy before jreg is reused
             continue;
@@ -501,11 +531,12 @@ klt_kernel_v3(const KltArgs a)
         __syncwarp();
 
         for (int j = 0; j < a.max_count; ++j) {
-            // nx, ny are finite here (finite inputs, bounded updates): F2I.FLOOR saturates where cvFloor gives INT_MIN,
-            // and both land on the same side of the range test
-            const int inx = __float2int_rd(nx), iny = __float2int_rd(ny);
-            unsigned ux = (unsigned)inx - (unsigned)xlo, uy = (unsigned)iny - (unsigned)ylo;
+            // cvFloor's INT_MIN, F2I's saturation and floor_v3 all land out of range where one of them does (floor_v3)
+            uint32_t bx, by;
+            const float fx = floor_v3(nx, bx), fy = floor_v3(ny, by);
+            unsigned ux = bx - xlob, uy = by - ylob;
             if (ux > xspan || uy > yspan) {
+                const int inx = floor_bits_to_int(bx), iny = floor_bits_to_int(by);
                 if (inx < -WW || inx >= lw || iny < -WH || iny >= lh) {
                     if (level == 0) st = 0;
                     break;
@@ -516,10 +547,10 @@ klt_kernel_v3(const KltArgs a)
                 cp_async_commit();
                 cp_async_wait_pending(0);
                 __syncwarp();
-                ux = (unsigned)inx - (unsigned)xlo; uy = (unsigned)iny - (unsigned)ylo;
+                ux = bx - xlob; uy = by - ylob;
             }
-            bilinear_weights(__fsub_rn(nx, (float)inx), __fsub_rn(ny, (float)iny), iw00, iw01, iw10, iw11);
-            const uint32_t jt = (uint32_t)(iw01 * 65536 + iw00), jb = (uint32_t)iw11 * 65536u + (uint32_t)iw10;
+            uint32_t jt, jb;
+            bilinear_weights_v3(__fsub_rn(nx, fx), __fsub_rn(ny, fy), jt, jb);
             const int joff = (int)uy * C::JS + (int)ux + jbase;
             int sb1 = -c1, sb2 = -c2;
             const int sh8 = (joff & 3) * 8;
@@ -563,23 +594,25 @@ klt_kernel_v3(const KltArgs a)
 
         if (st && level == 0) {
             const float qx = __fsub_rn(outx, hwx), qy = __fsub_rn(outy, hwy);
-            const int inx = floor_to_int(qx), iny = floor_to_int(qy);
+            uint32_t bx, by;
+            const float fx = floor_v3(qx, bx), fy = floor_v3(qy, by);
+            const int inx = floor_bits_to_int(bx), iny = floor_bits_to_int(by);
             if (inx < -WW || inx >= lw || iny < -WH || iny >= lh) {
                 st = 0;
                 continue;
             }
             if (!want_err) continue;
-            bilinear_weights(__fsub_rn(qx, (float)inx), __fsub_rn(qy, (float)iny), iw00, iw01, iw10, iw11);
-            unsigned ux = (unsigned)inx - (unsigned)xlo, uy = (unsigned)iny - (unsigned)ylo;
+            uint32_t jt, jb;
+            bilinear_weights_v3(__fsub_rn(qx, fx), __fsub_rn(qy, fy), jt, jb);
+            unsigned ux = bx - xlob, uy = by - ylob;
             if (ux > xspan || uy > yspan) {
                 __syncwarp();
                 stage_J(inx, iny);
                 cp_async_commit();
                 cp_async_wait_pending(0);
                 __syncwarp();
-                ux = (unsigned)inx - (unsigned)xlo; uy = (unsigned)iny - (unsigned)ylo;
+                ux = bx - xlob; uy = by - ylob;
             }
-            const uint32_t jt = (uint32_t)(iw01 * 65536 + iw00), jb = (uint32_t)iw11 * 65536u + (uint32_t)iw10;
             const int joff = (int)uy * C::JS + (int)ux + jbase;
             int se = 0;
 #pragma unroll
