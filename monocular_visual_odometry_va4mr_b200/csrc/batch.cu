@@ -1023,10 +1023,11 @@ extern "C" int b200vo_batch_good_features(b200vo_batch* B, int max_corners, doub
     VO_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     cudaEventElapsedTime(&ctx->last_ms, ctx->ev0, ctx->ev1);
     const int* small = (const int*)(hp + out_bytes);
-    for (int s = 0; s < nb; ++s) {
+    for (int s = 0; s < nb; ++s)   // every sequence is checked before any output is written: a refusal leaves them as they were
         if (small[s * VO_GFTT_SMALL + 1] > VO_GFTT_BATCH_CAP)
             return vo_set_err(ctx, B200VO_E_UNSUPPORTED, "sequence %d: %d corner candidates exceed the batched path's limit of %d (use the per-image call)",
                               s, small[s * VO_GFTT_SMALL + 1], VO_GFTT_BATCH_CAP);
+    for (int s = 0; s < nb; ++s) {
         const int n = small[s * VO_GFTT_SMALL + 2];
         n_corners[s] = n;
         memcpy(corners + (size_t)s * max_corners * 2, hp + (size_t)s * b_out, (size_t)n * 8);
