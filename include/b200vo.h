@@ -241,6 +241,24 @@ int b200vo_sift_detect_and_compute_masked(b200vo_ctx* ctx, const uint8_t* img, i
  */
 int b200vo_undistort(b200vo_ctx* ctx, const uint8_t* src, int rows, int cols, size_t step, const double K[9],
                      const double* dist, int n_dist, uint8_t* dst);
+/*
+ * Replaces cv2.undistort(src, K, dist, newCameraMatrix=Knew): as b200vo_undistort, with the undistorted image seen by the
+ * pinhole camera Knew (e.g. from cv2.getOptimalNewCameraMatrix) instead of K.  Knew == K is b200vo_undistort.
+ */
+int b200vo_undistort_new_camera(b200vo_ctx* ctx, const uint8_t* src, int rows, int cols, size_t step, const double K[9],
+                                const double* dist, int n_dist, const double Knew[9], uint8_t* dst);
+/* Lens models of the per-sequence lens (b200vo_batch_set_lens) */
+#define B200VO_LENS_PINHOLE 0   /* cv2's polynomial / rational model: k1, k2, p1, p2, k3, k4, k5, k6 */
+#define B200VO_LENS_FISHEYE 1   /* cv2.fisheye's equidistant model: k1, k2, k3, k4 */
+/*
+ * Replaces cv2.fisheye.undistortImage(src, K, D, Knew=Knew): src uint8 (rows, cols), `step` bytes a row; dst uint8 (rows,
+ * cols), tight.  K and Knew pinhole camera matrices, Knew == NULL the identity (as in cv2; usually the caller passes K or
+ * cv2.fisheye.estimateNewCameraMatrixForUndistortRectify's matrix); D double [4], finite.  Byte for byte what cv2
+ * computes: the map of cv2.fisheye.initUndistortRectifyMap(K, D, I, Knew, size, CV_16SC2), whose source pixel wraps
+ * modulo 2^16 as cv2 stores it, and a fixed-point bilinear remap with BORDER_CONSTANT 0.
+ */
+int b200vo_fisheye_undistort(b200vo_ctx* ctx, const uint8_t* src, int rows, int cols, size_t step, const double K[9],
+                             const double D[4], const double* Knew, uint8_t* dst);
 
 /*
  * Replaces cv2.solvePnPRansac(obj, img, K, zeros(4), flags=SOLVEPNP_P3P, confidence=,
@@ -330,6 +348,25 @@ int b200vo_batch_set_detection_mask(b200vo_batch* b, int n_seq, const int32_t* s
  * distortion; a batch without distortion builds its pyramids as it always did.  Synchronous.
  */
 int b200vo_batch_set_distortion(b200vo_batch* b, int n_seq, const int32_t* seqs, const double* dist);
+/*
+ * Per-sequence lens: b200vo_batch_set_distortion generalised to fisheye lenses and to raw cameras other than K.
+ * model: int32 [n_seq], B200VO_LENS_PINHOLE or B200VO_LENS_FISHEYE, or NULL: every row pinhole.  coeffs: double
+ * [n_seq][8], pinhole in cv2's order as b200vo_batch_set_distortion, fisheye k1, k2, k3, k4 in slots 0-3 and zeros in
+ * slots 4-7.  raw_K: double [n_seq][9], the
+ * pinhole camera the raw frames come from (the one the coefficients belong to), or NULL: the raw camera is the sequence's
+ * K.  The sequence's K (b200vo_batch_set_intrinsics) stays the camera of the undistorted image, which is what points,
+ * poses, masks and the bootstrap see: cv2.undistort(frame, raw_K, coeffs, newCameraMatrix=K) or
+ * cv2.fisheye.undistortImage(frame, raw_K, coeffs, Knew=K).  A sequence needs a map when it is fisheye (all-zero
+ * coefficients are the equidistant projection, not the identity), has a nonzero pinhole coefficient, or has a raw camera
+ * other than K; a pinhole row of zeros with raw_K NULL clears its lens.  b200vo_batch_set_intrinsics changes K and keeps
+ * an explicit raw camera; both it and b200vo_batch_set_frame_size rebuild the map.  b200vo_batch_set_distortion(dist) is
+ * this call with model NULL and raw_K NULL.  Bad indices (out of range, repeated), n_seq < 1, a null seqs or coeffs, an
+ * unknown model, a non-finite coefficient, a fisheye row with nonzero slots 4-7, a raw_K that is not a pinhole camera
+ * matrix, or submitted frame sets still waiting: B200VO_E_BADARG and nothing changes.  The resident frames no longer
+ * match: the next step needs b200vo_batch_prime.  Synchronous.
+ */
+int b200vo_batch_set_lens(b200vo_batch* b, int n_seq, const int32_t* seqs, const int32_t* model, const double* coeffs,
+                          const double* raw_K);
 /* Upload the first frame of every sequence (frames: batch x rows x cols, tight). */
 int b200vo_batch_prime(b200vo_batch* b, const uint8_t* frames);
 /*
@@ -434,6 +471,12 @@ int b200vo_loop_set_detection_mask(b200vo_loop* lp, int n_seq, const int32_t* se
  * the loaded state, keypoints, landmarks, poses, b200vo_loop_read_state and detection masks are in the undistorted image.
  * The listed sequences become B200VO_LOOP_IDLE until b200vo_loop_load or b200vo_loop_bootstrap runs for them.  Synchronous. */
 int b200vo_loop_set_distortion(b200vo_loop* lp, int n_seq, const int32_t* seqs, const double* dist);
+/* Per-sequence lens of the loop, as b200vo_batch_set_lens (same layout and validation: B200VO_E_BADARG, nothing changes).
+ * Every frame the loop takes is undistorted into the camera K of the sequence; b200vo_loop_set_intrinsics keeps an
+ * explicit raw camera.  The listed sequences become B200VO_LOOP_IDLE until b200vo_loop_load or b200vo_loop_bootstrap runs
+ * for them.  Synchronous. */
+int b200vo_loop_set_lens(b200vo_loop* lp, int n_seq, const int32_t* seqs, const int32_t* model, const double* coeffs,
+                         const double* raw_K);
 /* State of sequence `seq` after its bootstrap (host arrays): frame uint8 (rows,cols) tight at the sequence's own frame size
  * (b200vo_loop_set_frame_size) = the current frame;
  * lm float32 (n_lm,3) + lm_kp float32 (n_lm,2); keys / first_keys float32 (n_cand,2) + first_pose int32 (n_cand)

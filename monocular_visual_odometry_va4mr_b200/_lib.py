@@ -92,6 +92,8 @@ SIGNATURES = {
     "b200vo_sift_detect_and_compute_masked": (C.c_int, [C.c_void_p, c_u8p, C.c_int, C.c_int, C.c_size_t, c_u8p, C.c_size_t, C.c_int,
                                                         c_f32p, c_f32p, c_i32p]),
     "b200vo_undistort": (C.c_int, [C.c_void_p, c_u8p, C.c_int, C.c_int, C.c_size_t, c_f64p, c_f64p, C.c_int, c_u8p]),
+    "b200vo_undistort_new_camera": (C.c_int, [C.c_void_p, c_u8p, C.c_int, C.c_int, C.c_size_t, c_f64p, c_f64p, C.c_int, c_f64p, c_u8p]),
+    "b200vo_fisheye_undistort": (C.c_int, [C.c_void_p, c_u8p, C.c_int, C.c_int, C.c_size_t, c_f64p, c_f64p, c_f64p, c_u8p]),
     "b200vo_recover_pose": (C.c_int, [C.c_void_p, c_f64p, c_f32p, c_f32p, C.c_int, c_f64p, C.c_double, c_f64p, c_f64p, c_u8p, c_intp]),
     "b200vo_min_distance_mask": (C.c_int, [C.c_void_p, c_f32p, C.c_int, c_f32p, C.c_int, C.c_float, c_u8p]),
     "b200vo_triangulate_landmarks": (C.c_int, [
@@ -113,6 +115,7 @@ SIGNATURES = {
     "b200vo_batch_set_frame_size": (C.c_int, [C.c_void_p, C.c_int, c_i32p, c_i32p, c_i32p]),
     "b200vo_batch_set_detection_mask": (C.c_int, [C.c_void_p, C.c_int, c_i32p, c_u8p]),
     "b200vo_batch_set_distortion": (C.c_int, [C.c_void_p, C.c_int, c_i32p, c_f64p]),
+    "b200vo_batch_set_lens": (C.c_int, [C.c_void_p, C.c_int, c_i32p, c_i32p, c_f64p, c_f64p]),
     "b200vo_batch_prime": (C.c_int, [C.c_void_p, c_u8p]),
     "b200vo_batch_submit_frames": (C.c_int, [C.c_void_p, c_u8p]),
     "b200vo_batch_submit_frames_dev": (C.c_int, [C.c_void_p, C.c_void_p]),
@@ -129,6 +132,7 @@ SIGNATURES = {
     "b200vo_loop_set_frame_size": (C.c_int, [C.c_void_p, C.c_int, c_i32p, c_i32p, c_i32p]),
     "b200vo_loop_set_detection_mask": (C.c_int, [C.c_void_p, C.c_int, c_i32p, c_u8p]),
     "b200vo_loop_set_distortion": (C.c_int, [C.c_void_p, C.c_int, c_i32p, c_f64p]),
+    "b200vo_loop_set_lens": (C.c_int, [C.c_void_p, C.c_int, c_i32p, c_i32p, c_f64p, c_f64p]),
     "b200vo_loop_load": (C.c_int, [C.c_void_p, C.c_int, c_u8p, c_f32p, c_f32p, C.c_int, c_f32p, c_f32p, c_i32p, C.c_int, c_f64p,
                                    C.c_int]),
     "b200vo_loop_read_state": (C.c_int, [C.c_void_p, C.c_int, c_f32p, c_f32p, c_i32p, c_f32p, c_f32p, c_i32p, c_i32p, c_f64p, c_i32p,

@@ -88,8 +88,8 @@ class _PinnedBlock:
 class _Batch:
     """What SequenceBatch and VOBatch share: the C object of the functions ``<prefix>*`` (``b200vo_batch_`` or
     ``b200vo_loop_``) and its lifetime, page-locked arrays, and the settings every sequence has of its own -- camera
-    matrix, frame size, detection mask and lens distortion -- with their host mirrors ``frame_size``, ``has_mask`` and
-    ``dist_coeffs``."""
+    matrix, frame size, detection mask and lens -- with their host mirrors ``frame_size``, ``has_mask``, ``dist_coeffs``,
+    ``dist_model`` and ``raw_K``."""
 
     def __init__(self, prefix, batch, rows, cols, ctx):
         self._prefix = prefix
@@ -98,10 +98,12 @@ class _Batch:
         self.frame_size = np.tile(np.int32([self.rows, self.cols]), (self.batch, 1))   # (batch, 2) rows, cols of every sequence
         self.has_mask = np.zeros(self.batch, bool)   # the sequences with a detection mask (set_detection_mask)
         self.dist_coeffs = np.zeros((self.batch, 8))   # k1, k2, p1, p2, k3, k4, k5, k6 of every sequence (set_distortion)
+        self.dist_model = np.full(self.batch, "pinhole", "<U7")   # "pinhole" or "fisheye" (k1 .. k4 in dist_coeffs[:, :4])
+        self.raw_K = np.full((self.batch, 3, 3), np.nan)   # the raw cameras set by set_distortion; NaN: the sequence's K
         self._submitted = []   # page-locked slot-layout copies of submitted frame lists, alive until their step
 
-    def _create(self, cfg, K_rows, frame_size, dist_coeffs):
-        """Creates the C object from ``cfg``, then applies the constructor's per-sequence K rows, frame sizes and distortion."""
+    def _create(self, cfg, K_rows, frame_size, dist_coeffs, dist_model="pinhole", raw_K=None):
+        """Creates the C object from ``cfg``, then applies the constructor's per-sequence K rows, frame sizes and lenses."""
         self.cfg = cfg
         h = C.c_void_p()
         rc = getattr(self.ctx.lib, self._prefix + "create")(self.ctx.h, self.batch, C.byref(cfg), C.byref(h))
@@ -112,8 +114,8 @@ class _Batch:
             self.set_intrinsics(np.arange(self.batch), K_rows)
         if frame_size is not None:
             self.set_frame_size(np.arange(self.batch), frame_size)
-        if dist_coeffs is not None:
-            self.set_distortion(np.arange(self.batch), dist_coeffs)
+        if dist_coeffs is not None or raw_K is not None or not np.all(np.asarray(dist_model) == "pinhole"):
+            self.set_distortion(np.arange(self.batch), dist_coeffs, dist_model, raw_K)
 
     def close(self):
         """Destroys the device-side object.  Page-locked arrays handed out by this object (step() results,
@@ -161,8 +163,8 @@ class _Batch:
     def set_intrinsics(self, seqs, K):
         """Give the distinct sequences ``seqs`` the camera matrices ``K`` (len(seqs), 3, 3); everything later that poses,
         triangulates or undistorts those sequences uses their own K.  A K must be a pinhole camera: fx, fy finite and > 0,
-        cx, cy finite, zero skew and other off-diagonal entries, last row (0, 0, 1).  A sequence with distortion keeps its
-        coefficients and gets a new map; its K cannot change while submitted frames wait.  Bad shapes, indices or matrices
+        cx, cy finite, zero skew and other off-diagonal entries, last row (0, 0, 1).  A sequence with a lens keeps its
+        lens and raw camera (``raw_K``) and gets a new map; its K cannot change while submitted frames wait.  Bad shapes, indices or matrices
         raise ValueError and change nothing.  Synchronous."""
         seqs = np.ascontiguousarray(seqs, np.int32).reshape(-1)
         K = np.ascontiguousarray(K, np.float64)
@@ -174,7 +176,7 @@ class _Batch:
         """Give the distinct sequences ``seqs`` the frame sizes ``sizes`` (len(seqs), 2) int (rows, cols).  ``rows`` x ``cols`` of the
         constructor is the slot, the largest frame: a sequence's image is the top-left of its slot in every frame array (which
         may also be a list of per-sequence images), and each sequence runs exactly as in a batch of its own size.  A size must
-        fit the slot and exceed the window.  The listed sequences lose their detection masks and keep their distortion, with
+        fit the slot and exceed the window.  The listed sequences lose their detection masks and keep their lenses, with
         new maps.  Bad shapes, indices or sizes, or submitted frames still waiting, raise ValueError and change nothing.
         Synchronous."""
         seqs = np.ascontiguousarray(seqs, np.int32).reshape(-1)
@@ -206,25 +208,53 @@ class _Batch:
         self._call("set_detection_mask", len(seqs), _p(seqs, c_i32p), None if masks is None else _p(masks, c_u8p))
         self.has_mask[seqs] = masks is not None
 
-    def set_distortion(self, seqs, dist):
-        """Give the distinct sequences ``seqs`` lens distortion: ``dist`` (len(seqs), n) with n = 4, 5 or 8 coefficients in cv2's
-        order (k1, k2, p1, p2[, k3[, k4, k5, k6]]), or None to clear it; an all-zero row clears it too.  Every frame of a
-        sequence with distortion is raw camera output, undistorted on the device as ``cv2.undistort(frame, K, dist)`` does
-        (``cv2_compat.undistort``) before anything reads it: points, poses, states, detected corners and detection masks are in
-        the undistorted image, whose camera is the sequence's K.  ``set_intrinsics`` and ``set_frame_size`` keep the
-        coefficients and rebuild the map.  Bad shapes, non-finite coefficients, bad indices or submitted frames still waiting
-        raise ValueError (the 12- and 14-coefficient models NotImplementedError) and change nothing.  Synchronous."""
+    def set_distortion(self, seqs, dist, model="pinhole", raw_K=None):
+        """Give the distinct sequences ``seqs`` a lens.  ``model`` is "pinhole" or "fisheye", for all of them or one per
+        sequence.  ``dist`` (len(seqs), n) holds the coefficients in cv2's order, or None for zeros: a pinhole lens takes
+        n = 4, 5 or 8 (k1, k2, p1, p2[, k3[, k4, k5, k6]]), a fisheye lens the 4 of ``cv2.fisheye`` (k1, k2, k3, k4; in a call
+        that mixes models, a fisheye row's columns after the fourth are 0).  ``raw_K`` (len(seqs), 3, 3): the pinhole cameras
+        the raw frames come from, which the coefficients belong to; None: the sequences' own K.  Every frame of a sequence
+        with a lens is raw camera output, undistorted on the device before anything reads it, as
+        ``cv2.undistort(frame, raw_K, dist, newCameraMatrix=K)`` or ``cv2.fisheye.undistortImage(frame, raw_K, dist, Knew=K)``
+        do (``cv2_compat.undistort``, ``cv2_compat.fisheye_undistort_image``): points, poses, states, detected corners and
+        detection masks are in the undistorted image, whose camera is the sequence's K.  A pinhole lens with all-zero
+        coefficients and no ``raw_K`` clears it; a fisheye lens with zero coefficients is the equidistant projection.
+        ``set_intrinsics`` changes K, keeps an explicit ``raw_K``, and rebuilds the map, as ``set_frame_size`` does.  Bad
+        shapes, models, non-finite coefficients, a ``raw_K`` that is not a pinhole camera, bad indices or submitted frames
+        still waiting raise ValueError (the 12- and 14-coefficient models NotImplementedError) and change nothing.
+        Synchronous."""
         seqs = self._seqs(seqs)
-        d8 = np.zeros((len(seqs), 8), np.float64)
+        n = len(seqs)
+        models = np.broadcast_to(np.asarray(model), (n,)) if np.ndim(model) <= 1 and np.size(model) in (1, n) else None
+        if models is None or not np.isin(models, ("pinhole", "fisheye")).all():
+            raise ValueError(f'model must be "pinhole" or "fisheye", or one of them per sequence, got {model!r}')
+        fisheye = models == "fisheye"
+        d8 = np.zeros((n, 8), np.float64)
         if dist is not None:
             d = np.asarray(dist)
-            if d.ndim == 2 and d.shape[0] == len(seqs) and d.shape[1] in (12, 14):
-                raise NotImplementedError("the thin-prism (12) and tilted (14) distortion models are not supported")
-            if d.ndim != 2 or d.shape[0] != len(seqs) or d.shape[1] not in (4, 5, 8) or not np.issubdtype(d.dtype, np.number):
-                raise ValueError(f"dist must be (len(seqs) = {len(seqs)}, 4 | 5 | 8) coefficients or None, got {d.dtype} {d.shape}")
+            if fisheye.all():
+                if d.ndim != 2 or d.shape != (n, 4) or not np.issubdtype(d.dtype, np.number):
+                    raise ValueError(f"a fisheye dist must be (len(seqs) = {n}, 4) coefficients or None, got {d.dtype} {d.shape}")
+            else:
+                if d.ndim == 2 and d.shape[0] == n and d.shape[1] in (12, 14):
+                    raise NotImplementedError("the thin-prism (12) and tilted (14) distortion models are not supported")
+                if d.ndim != 2 or d.shape[0] != n or d.shape[1] not in (4, 5, 8) or not np.issubdtype(d.dtype, np.number):
+                    raise ValueError(f"dist must be (len(seqs) = {n}, 4 | 5 | 8) coefficients or None, got {d.dtype} {d.shape}")
             d8[:, :d.shape[1]] = d
-        self._call("set_distortion", len(seqs), _p(seqs, c_i32p), _p(d8, c_f64p))
+        raw = None
+        if raw_K is not None:
+            raw = np.ascontiguousarray(raw_K, np.float64)
+            if raw.shape != (n, 3, 3):
+                raise ValueError(f"raw_K must be (len(seqs) = {n}, 3, 3) or None, got {raw.shape}")
+        code = np.ascontiguousarray(fisheye, np.int32)
+        self._call("set_lens", n, _p(seqs, c_i32p), _p(code, c_i32p), _p(d8, c_f64p), None if raw is None else _p(raw, c_f64p))
         self.dist_coeffs[seqs] = d8
+        self.dist_model[seqs] = models
+        self.raw_K[seqs] = np.nan if raw is None else raw
+
+    def _needs_map(self, seq) -> bool:
+        """whether sequence ``seq``'s frames may go through a map that depends on its K"""
+        return bool(self.dist_model[seq] == "fisheye" or self.dist_coeffs[seq].any() or not np.isnan(self.raw_K[seq]).all())
 
 
 class SequenceBatch(_Batch):
@@ -236,7 +266,8 @@ class SequenceBatch(_Batch):
 
     def __init__(self, batch, rows, cols, K, win=(15, 15), max_level=5, criteria=(3, 50, 0.01),
                  min_eig_thr=1e-4, pnp_iters=500, pnp_reproj_err=8.0, pnp_conf=0.99,
-                 max_landmarks=1024, max_candidates=1024, frame_size=None, dist_coeffs=None, ctx: _lib.Context | None = None):
+                 max_landmarks=1024, max_candidates=1024, frame_size=None, dist_coeffs=None, dist_model="pinhole", raw_K=None,
+                 ctx: _lib.Context | None = None):
         super().__init__("b200vo_batch_", batch, rows, cols, ctx)
         self.L, self.Cn = int(max_landmarks), int(max_candidates)
         cfg = BatchCfg()
@@ -250,7 +281,7 @@ class SequenceBatch(_Batch):
         for i in range(9):
             cfg.K[i] = float(Kf[i])
         cfg.max_landmarks, cfg.max_candidates = self.L, self.Cn
-        self._create(cfg, K_rows, frame_size, dist_coeffs)
+        self._create(cfg, K_rows, frame_size, dist_coeffs, dist_model, raw_K)
         # host outputs (reused, page-locked so that step() reads them back without a staging copy)
         b, L, Cn = self.batch, self.L, self.Cn
         self.lm_next = self.pinned_empty((b, L, 2), np.float32)
@@ -392,12 +423,13 @@ class VOBatch(_Batch):
     OK, IDLE, FEW_POINTS, PNP_FAILED, OVERFLOW, DETECT_LIMIT, NO_BOOTSTRAP = range(7)
 
     def __init__(self, batch, rows, cols, K, options, max_landmarks=4096, max_candidates=8192, max_frames=1024,
-                 frame_size=None, dist_coeffs=None, ctx: _lib.Context | None = None):
+                 frame_size=None, dist_coeffs=None, dist_model="pinhole", raw_K=None, ctx: _lib.Context | None = None):
         super().__init__("b200vo_loop_", batch, rows, cols, ctx)
         self.L, self.Cn, self.P = int(max_landmarks), int(max_candidates), int(max_frames)
         self.options = options
         K, K_rows = _batch_K(K, self.batch)
-        self._create(_loop_cfg(rows, cols, K, options, max_landmarks, max_candidates, max_frames), K_rows, frame_size, dist_coeffs)
+        self._create(_loop_cfg(rows, cols, K, options, max_landmarks, max_candidates, max_frames), K_rows, frame_size, dist_coeffs,
+                     dist_model, raw_K)
         b = self.batch
         self._res = dict(status=self.pinned_empty((b,), np.int32), n_inliers=self.pinned_empty((b,), np.int32),
                          n_lm=self.pinned_empty((b,), np.int32), n_cand=self.pinned_empty((b,), np.int32),
@@ -428,9 +460,9 @@ class VOBatch(_Batch):
             K = np.asarray(K, np.float64)
             if K.shape != (3, 3) or not _pinhole(K):
                 raise ValueError("K must be a (3, 3) pinhole camera matrix (see set_intrinsics)")
-        K_first = K is not None and bool(self.dist_coeffs[int(seq)].any())
+        K_first = K is not None and self._needs_map(int(seq))
         if K_first:
-            # the frame is undistorted with the sequence's K: it must be in place before the load, so the load's own
+            # the frame is undistorted into the sequence's K: it must be in place before the load, so the load's own
             # refusals are checked here first to leave everything unchanged on bad input
             if not (len(lm) <= self.L and len(keys) <= self.Cn and 1 <= len(poses) <= self.P) or (fp < 0).any() or (fp >= len(poses)).any():
                 raise ValueError("b200vo_loop_load: a count is out of range or a first_pose value outside [0, n_poses)")
@@ -448,7 +480,7 @@ class VOBatch(_Batch):
         arrays (len(seqs),): ``status`` (OK, NO_BOOTSTRAP or OVERFLOW), ``num_pts`` (the essential-matrix inlier count),
         ``n_lm`` and ``n_cand``.  A failing sequence keeps its state and is skipped by ``step`` until it is loaded or
         bootstrapped again.  ``K`` (len(seqs), 3, 3): the listed sequences' cameras from now on (``set_intrinsics`` first).
-        A sequence with distortion (``set_distortion``) runs on its undistorted frames: it ends up as ``load(s, frames1[k],
+        A sequence with a lens (``set_distortion``) runs on its undistorted frames, and ``K`` keeps its raw camera: it ends up as ``load(s, frames1[k],
         initial_state(K, options, *match_bootstrap_frames(undistort(frames0[k]), undistort(frames1[k]), ratio)))`` leaves it.
         Bad indices, frame shapes or K raise ValueError and change nothing.  Synchronous."""
         seqs = np.arange(self.batch, dtype=np.int32) if seqs is None else np.ascontiguousarray(seqs, np.int32).reshape(-1)

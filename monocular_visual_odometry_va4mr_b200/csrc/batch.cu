@@ -50,49 +50,51 @@ scatter_mask_kernel(int cap, const uint8_t* __restrict__ ok, const int* __restri
     if (threadIdx.x == 0) { n_inl_out[b] = m; ok_out[b] = ok[b]; }
 }
 
-enum VoSetting { VO_SET_INTRINSICS, VO_SET_FRAME_SIZE, VO_SET_DISTORTION, VO_SET_MASK };
+enum VoSetting { VO_SET_INTRINSICS, VO_SET_FRAME_SIZE, VO_SET_LENS, VO_SET_MASK };
 
 // What a new setting of the listed sequences does besides writing their rows.  A submitted frame set's pyramids were built
 // (and undistorted) with the settings of its submission: `waiting` is the refusal while one waits (nullptr: never refused;
-// only_distorted: only when a listed sequence has distortion, the one use of K in a pyramid).  stale: the listed sequences'
+// only_mapped: only when a listed sequence needs a map, the one use of K in a pyramid).  stale: the listed sequences'
 // resident pyramids no longer match their frames.  unmask: a mask has its sequence's frame size, so the listed sequences
-// lose theirs.  remap: a map depends on K, the coefficients and the frame size, so the listed sequences with distortion
-// get new maps (their coefficients kept).
-static const struct { const char* waiting; bool only_distorted, stale, unmask, remap; } k_setting[] = {
+// lose theirs.  remap: a map depends on K, the lens and the frame size, so the listed sequences that need one get new
+// maps (their lenses kept).
+static const struct { const char* waiting; bool only_mapped, stale, unmask, remap; } k_setting[] = {
     /* intrinsics */     {"submitted frame sets are waiting: their pyramids were undistorted with the old K", true, false, false, true},
     /* frame size */     {"submitted frame sets are waiting: their pyramids were built at the old sizes", false, true, true, true},
-    /* distortion */     {"submitted frame sets are waiting: their pyramids were built with the old maps", false, true, false, true},
+    /* lens */           {"submitted frame sets are waiting: their pyramids were built with the old maps", false, true, false, true},
     /* detection mask */ {nullptr, false, false, false, false},
 };
 
-// the map of every listed sequence with distortion, from its K, coefficients and frame size (the work in flight has ended)
+// the map of every listed sequence that needs one, from its lens, raw camera, K and frame size (the work in flight has
+// ended): one launch per lens model
 static int batch_build_maps(b200vo_batch* B, int n_seq, const int32_t* seqs)
 {
     b200vo_ctx* ctx = B->ctx;
     const b200vo_batch_cfg& c = B->cfg;
-    std::vector<double> par;
-    std::vector<int32_t> im;
-    for (int k = 0; k < n_seq; ++k) {
-        const int s = seqs[k];
-        const VoSeqSettings& q = B->seq[s];
-        if (!q.distorted()) continue;
-        const VoIntrinsics& r = q.intr;
-        const double* d = q.dist;
-        const double row[14] = {r.fx, r.fy, r.cx, r.cy, d[0], d[1], d[2], d[3], d[4], d[5], d[6], d[7],
-                                (double)q.ext.w[0], (double)q.ext.h[0]};
-        par.insert(par.end(), row, row + 14);
-        im.push_back(s);
-    }
-    if (im.empty()) return 0;
-    const size_t n = im.size(), b_par = vo_align(n * 14 * sizeof(double), 256), fb = (size_t)c.rows * c.cols;
-    VO_TRY(vo_reserve(ctx, B->dist_par, b_par + n * 4));
-    uint8_t* p = (uint8_t*)B->dist_par.p;
-    VO_CUDA(ctx, cudaMemcpyAsync(p, par.data(), par.size() * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
-    VO_CUDA(ctx, cudaMemcpyAsync(p + b_par, im.data(), n * 4, cudaMemcpyHostToDevice, ctx->stream));
+    const size_t fb = (size_t)c.rows * c.cols;
     uint8_t* m = (uint8_t*)B->dist_buf.p + vo_align((size_t)B->batch, 256);
-    VO_TRY(vo_undistort_maps(ctx, (const double*)p, (const int*)(p + b_par), (int)n, c.rows, c.cols, (short2*)m,
-                             (uint16_t*)(m + (size_t)B->batch * fb * 4), fb, c.cols, ctx->stream));
-    VO_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    for (int model : {B200VO_LENS_PINHOLE, B200VO_LENS_FISHEYE}) {
+        std::vector<double> par;
+        std::vector<int32_t> im;
+        for (int k = 0; k < n_seq; ++k) {
+            const int s = seqs[k];
+            const VoSeqSettings& q = B->seq[s];
+            if (!q.needs_map() || q.model != model) continue;
+            double row[VO_LENS_PAR];
+            vo_lens_row(row, q.raw_set ? q.raw : q.intr, q.intr, q.dist, q.ext.w[0], q.ext.h[0]);
+            par.insert(par.end(), row, row + VO_LENS_PAR);
+            im.push_back(s);
+        }
+        if (im.empty()) continue;
+        const size_t n = im.size(), b_par = vo_align(n * VO_LENS_PAR * sizeof(double), 256);
+        VO_TRY(vo_reserve(ctx, B->dist_par, b_par + n * 4));
+        uint8_t* p = (uint8_t*)B->dist_par.p;
+        VO_CUDA(ctx, cudaMemcpyAsync(p, par.data(), par.size() * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+        VO_CUDA(ctx, cudaMemcpyAsync(p + b_par, im.data(), n * 4, cudaMemcpyHostToDevice, ctx->stream));
+        VO_TRY(vo_undistort_maps(ctx, model, (const double*)p, (const int*)(p + b_par), (int)n, c.rows, c.cols, (short2*)m,
+                                 (uint16_t*)(m + (size_t)B->batch * fb * 4), fb, c.cols, ctx->stream));
+        VO_CUDA(ctx, cudaStreamSynchronize(ctx->stream));   // the parameter rows are reused by the next model
+    }
     return 0;
 }
 
@@ -106,9 +108,11 @@ static int batch_apply(b200vo_batch* B, VoSetting kind, std::vector<VoSeqSetting
     const b200vo_batch_cfg& c = B->cfg;
     const int nb = B->batch;
     const auto& rule = k_setting[kind];
-    bool listed_dist = false;
-    for (int k = 0; k < n_seq; ++k) listed_dist = listed_dist || next[seqs[k]].distorted();
-    if (rule.waiting && B->q_count > 0 && (!rule.only_distorted || listed_dist)) return vo_set_err(ctx, B200VO_E_BADARG, "%s", rule.waiting);
+    if (rule.waiting && B->q_count > 0) {   // (a batch being created has no table yet, and nothing submitted)
+        bool listed_map = false;   // before or after: a set built with a map, or without one, no longer matches
+        for (int k = 0; k < n_seq; ++k) listed_map = listed_map || B->seq[seqs[k]].needs_map() || next[seqs[k]].needs_map();
+        if (!rule.only_mapped || listed_map) return vo_set_err(ctx, B200VO_E_BADARG, "%s", rule.waiting);
+    }
     if (rule.unmask)
         for (int k = 0; k < n_seq; ++k) next[seqs[k]].mask = false;
     std::vector<VoIntrinsics> intr(nb);
@@ -120,7 +124,7 @@ static int batch_apply(b200vo_batch* B, VoSetting kind, std::vector<VoSeqSetting
         intr[s] = next[s].intr;
         ext[s] = next[s].ext;
         mask_flag[s] = next[s].mask;
-        dist_flag[s] = next[s].distorted();
+        dist_flag[s] = next[s].needs_map();
         n_mask += mask_flag[s];
         n_dist += dist_flag[s];
         uniform = uniform && ext[s].w[0] == c.cols && ext[s].h[0] == c.rows;
@@ -214,7 +218,7 @@ extern "C" int b200vo_batch_create(b200vo_ctx* ctx, int batch, const b200vo_batc
     B->inliers = (int*)p; p += b_i;
     B->c_mask = p; p += b_m;
     B->pnp_ws = p;
-    // every sequence starts with cfg->K, the slot size, no mask and no distortion (no mask or map buffer until the first one)
+    // every sequence starts with cfg->K, the slot size, no mask and no lens (no mask or map buffer until the first one)
     std::vector<VoSeqSettings> table(batch, VoSeqSettings{});
     vo_intrinsics_row(table[0].intr, cfg->K, VO_BOOT_EMAT_THR);
     vo_seq_ext(cfg->rows, cfg->cols, cfg->win_w, cfg->win_h, cfg->max_level, &table[0].ext);
@@ -261,16 +265,32 @@ int batch_set_frame_size(b200vo_batch* B, int n_seq, const int32_t* seqs, const 
     return batch_apply(B, VO_SET_FRAME_SIZE, next, n_seq, seqs, nullptr, stale);
 }
 
-int batch_set_distortion(b200vo_batch* B, int n_seq, const int32_t* seqs, const double* dist, bool* stale)
+int batch_set_lens(b200vo_batch* B, int n_seq, const int32_t* seqs, const int32_t* model, const double* coeffs, const double* raw_K,
+                   bool* stale)
 {
     b200vo_ctx* ctx = B->ctx;
     VO_TRY(vo_check_seqs(ctx, B->batch, n_seq, seqs));
-    if (!dist) return vo_set_err(ctx, B200VO_E_BADARG, "null array");
-    for (int k = 0; k < n_seq; ++k)
-        if (!vo_dist_valid(dist + 8 * (size_t)k)) return vo_set_err(ctx, B200VO_E_BADARG, "sequence %d: non-finite distortion coefficient", seqs[k]);
+    if (!coeffs) return vo_set_err(ctx, B200VO_E_BADARG, "null array");
+    for (int k = 0; k < n_seq; ++k) {
+        const double* d = coeffs + 8 * (size_t)k;
+        const int mk = model ? model[k] : B200VO_LENS_PINHOLE;
+        if (mk != B200VO_LENS_PINHOLE && mk != B200VO_LENS_FISHEYE)
+            return vo_set_err(ctx, B200VO_E_BADARG, "sequence %d: unknown lens model %d", seqs[k], mk);
+        if (!vo_dist_valid(d)) return vo_set_err(ctx, B200VO_E_BADARG, "sequence %d: non-finite distortion coefficient", seqs[k]);
+        if (mk == B200VO_LENS_FISHEYE && (d[4] != 0 || d[5] != 0 || d[6] != 0 || d[7] != 0))
+            return vo_set_err(ctx, B200VO_E_BADARG, "sequence %d: a fisheye lens has 4 coefficients (slots 4-7 must be 0)", seqs[k]);
+        if (raw_K && !vo_intrinsics_valid(raw_K + 9 * (size_t)k))
+            return vo_set_err(ctx, B200VO_E_BADARG, "sequence %d: raw_K is not a pinhole camera matrix", seqs[k]);
+    }
     std::vector<VoSeqSettings> next = B->seq;
-    for (int k = 0; k < n_seq; ++k) memcpy(next[seqs[k]].dist, dist + 8 * (size_t)k, 8 * sizeof(double));
-    return batch_apply(B, VO_SET_DISTORTION, next, n_seq, seqs, nullptr, stale);
+    for (int k = 0; k < n_seq; ++k) {
+        VoSeqSettings& q = next[seqs[k]];
+        q.model = model ? model[k] : B200VO_LENS_PINHOLE;
+        memcpy(q.dist, coeffs + 8 * (size_t)k, 8 * sizeof(double));
+        q.raw_set = raw_K != nullptr;
+        if (raw_K) vo_intrinsics_row(q.raw, raw_K + 9 * (size_t)k, VO_BOOT_EMAT_THR);
+    }
+    return batch_apply(B, VO_SET_LENS, next, n_seq, seqs, nullptr, stale);
 }
 
 int batch_set_detection_mask(b200vo_batch* B, int n_seq, const int32_t* seqs, const uint8_t* masks, bool* stale)
@@ -285,7 +305,7 @@ VoUndist batch_undist(const b200vo_batch* B, int b0, int n, const int32_t* list)
 {
     VoUndist u;
     bool any = false;
-    for (int k = 0; B->n_dist && !any && k < n; ++k) any = B->seq[list ? list[k] : b0 + k].distorted();
+    for (int k = 0; B->n_dist && !any && k < n; ++k) any = B->seq[list ? list[k] : b0 + k].needs_map();
     if (!any) return u;
     const size_t fb = (size_t)B->cfg.rows * B->cfg.cols;
     const uint8_t* d = (const uint8_t*)B->dist_buf.p;
@@ -340,7 +360,16 @@ extern "C" int b200vo_batch_set_frame_size(b200vo_batch* B, int n_seq, const int
 extern "C" int b200vo_batch_set_distortion(b200vo_batch* B, int n_seq, const int32_t* seqs, const double* dist)
 {
     bool stale = false;
-    const int rc = B ? batch_set_distortion(B, n_seq, seqs, dist, &stale) : B200VO_E_BADARG;
+    const int rc = B ? batch_set_lens(B, n_seq, seqs, nullptr, dist, nullptr, &stale) : B200VO_E_BADARG;
+    if (stale) B->primed = false;
+    return rc;
+}
+
+extern "C" int b200vo_batch_set_lens(b200vo_batch* B, int n_seq, const int32_t* seqs, const int32_t* model, const double* coeffs,
+                                     const double* raw_K)
+{
+    bool stale = false;
+    const int rc = B ? batch_set_lens(B, n_seq, seqs, model, coeffs, raw_K, &stale) : B200VO_E_BADARG;
     if (stale) B->primed = false;
     return rc;
 }

@@ -9,18 +9,23 @@
 // host-buffer steps whose point arrays and results together stay below this go up / come back as ONE copy each
 #define B200VO_PACKED_IO_BYTES (512 * 1024)
 
-// One sequence's settings as the host keeps them (b200vo_batch_set_intrinsics / _frame_size / _detection_mask /
-// _distortion); the device holds their forms the kernels read (b200vo_batch::intr_buf, ext_buf, mask_buf, dist_buf)
+// One sequence's settings as the host keeps them (b200vo_batch_set_intrinsics / _frame_size / _detection_mask / _lens);
+// the device holds their forms the kernels read (b200vo_batch::intr_buf, ext_buf, mask_buf, dist_buf)
 struct VoSeqSettings {
-    VoIntrinsics intr;
+    VoIntrinsics intr;   // K: the camera of the undistorted image
     VoSeqExt ext;
-    double dist[8];   // k1, k2, p1, p2, k3, k4, k5, k6; all zero: no distortion
-    bool mask;        // has a detection mask
-    bool distorted() const
+    int model;           // B200VO_LENS_PINHOLE / B200VO_LENS_FISHEYE
+    double dist[8];      // pinhole: k1, k2, p1, p2, k3, k4, k5, k6; fisheye: k1 .. k4, 0, 0, 0, 0
+    bool raw_set;        // raw: the camera of the raw frames; unset: it is K
+    VoIntrinsics raw;
+    bool mask;           // has a detection mask
+    // the raw frames are undistorted through a map: a fisheye lens, a pinhole coefficient or a raw camera other than K
+    bool needs_map() const
     {
+        if (model == B200VO_LENS_FISHEYE) return true;
         for (double d : dist)
             if (d != 0.0) return true;
-        return false;
+        return raw_set && (raw.fx != intr.fx || raw.fy != intr.fy || raw.cx != intr.cx || raw.cy != intr.cy);
     }
 };
 
@@ -67,13 +72,13 @@ struct b200vo_batch {
     void* pnp_ws;
     const uint32_t* rng; int n_raw;
     bool primed;
-    // the settings of every sequence (batch_apply): the host table, how many sequences have a mask / distortion, and the
+    // the settings of every sequence (batch_apply): the host table, how many sequences have a mask / a map, and the
     // device forms.  intr_buf: the VoIntrinsics rows.  ext_buf: the VoSeqExt rows, read by the pyramid, tracker and detector
     // kernels; `ext` is nullptr while every sequence has the slot size cfg.rows x cfg.cols: the kernels then take the slot
     // geometry from their launch arguments, as a batch without per-sequence sizes always did.  mask_buf: [batch] "has a
-    // mask" bytes, then [batch] masks in the slot layout, allocated with the first mask.  dist_buf: [batch] "has distortion"
+    // mask" bytes, then [batch] masks in the slot layout, allocated with the first mask.  dist_buf: [batch] "has a map"
     // bytes, then [batch] int16 source-pixel maps and [batch] uint16 fraction maps in the slot layout (VoUndist), allocated
-    // with the first distortion.  n_mask == 0: the detectors get no mask; n_dist == 0: pyramids as without distortion.
+    // with the first map.  n_mask == 0: the detectors get no mask; n_dist == 0: pyramids as without distortion.
     std::vector<VoSeqSettings> seq;
     int n_mask = 0, n_dist = 0;
     DevBuf intr_buf;
@@ -124,11 +129,13 @@ int batch_set_intrinsics(b200vo_batch* B, int n_seq, const int32_t* seqs, const 
 int batch_set_frame_size(b200vo_batch* B, int n_seq, const int32_t* seqs, const int32_t* rows, const int32_t* cols, bool* stale);
 // masks: uint8 [n_seq][cfg.rows][cfg.cols], nullptr: the listed sequences' masks are cleared
 int batch_set_detection_mask(b200vo_batch* B, int n_seq, const int32_t* seqs, const uint8_t* masks, bool* stale);
-// dist: [n_seq][8] k1, k2, p1, p2, k3, k4, k5, k6; an all-zero row clears a sequence's distortion
-int batch_set_distortion(b200vo_batch* B, int n_seq, const int32_t* seqs, const double* dist, bool* stale);
+// model: [n_seq] B200VO_LENS_*, nullptr: all pinhole; coeffs: [n_seq][8]; raw_K: [n_seq][9] or nullptr (the raw camera is
+// K); a pinhole all-zero row without raw_K clears a sequence's lens
+int batch_set_lens(b200vo_batch* B, int n_seq, const int32_t* seqs, const int32_t* model, const double* coeffs, const double* raw_K,
+                   bool* stale);
 // the masks of the detectors: indexed by sequence, none while no sequence has one
 VoMask batch_mask(const b200vo_batch* B);
-// the maps of sequences b0 .. b0 + n - 1, or of the n sequences list[k] (b0 == 0); none while none of them has distortion
+// the maps of sequences b0 .. b0 + n - 1, or of the n sequences list[k] (b0 == 0); none while none of them needs one
 VoUndist batch_undist(const b200vo_batch* B, int b0, int n, const int32_t* list = nullptr);
 // The pyramids of n raw images (device, slot layout, one slot apart) into slab set `set`, each at its sequence's extents
 // and with its map: image k is sequence b0 + k, or with a list (its device row and host copy, b0 == 0) sequence list[k]

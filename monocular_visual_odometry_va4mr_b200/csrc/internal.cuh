@@ -50,9 +50,10 @@ struct VoMask {
     int pitch = 0;
 };
 
-// Lens distortion (cv2.undistort with newCameraMatrix = K): image im's fixed-point map in cv2's CV_16SC2 + CV_16UC1
-// layout, entry (x, y) at im * stride + y * pitch + x: xy = the source pixel (saturated to int16), fr = (v & 31) * 32 +
-// (u & 31) in 1/32 px.  on[im] == 0: image im has no distortion (copied as is); on == nullptr: every image has one.
+// Lens distortion (cv2.undistort, cv2.fisheye.undistortImage): image im's fixed-point map in cv2's CV_16SC2 + CV_16UC1
+// layout, entry (x, y) at im * stride + y * pitch + x: xy = the source pixel (int16, saturated or wrapped as the lens
+// model's cv2 map stores it), fr = (v & 31) * 32 + (u & 31) in 1/32 px.  on[im] == 0: image im has no map (copied as is);
+// on == nullptr: every image has one.
 // xy == nullptr: no image of the launch has distortion, and the pyramid builder runs exactly as without this argument.
 struct VoUndist {
     const short2* xy = nullptr;
@@ -217,12 +218,18 @@ int vo_build_pyramids(b200vo_ctx* ctx, const uint8_t* d_raw, size_t raw_stride, 
                       const int* d_list = nullptr, const int* h_list = nullptr, int n_slab = 0, const VoUndist& ud = VoUndist{});
 
 // ---- undistort.cu ----
-// The 8 coefficients k1, k2, p1, p2, k3, k4, k5, k6 are finite (what *_set_distortion and b200vo_undistort accept)
+// The 8 coefficients k1, k2, p1, p2, k3, k4, k5, k6 (fisheye: k1 .. k4, then zeros) are finite (what the lens setters and
+// the one-call forms accept)
 bool vo_dist_valid(const double d[8]);
-// map of image im = 0 .. n-1 (cv2.initUndistortRectifyMap(K, d, None, K, (cols[im], rows[im]), CV_16SC2)) into
-// xy / fr + im_of[im] * stride, rows `pitch` entries apart.  par: [n][14] doubles fx, fy, cx, cy, k1 .. k6, cols, rows.
-int vo_undistort_maps(b200vo_ctx* ctx, const double* d_par, const int* d_im_of, int n, int max_rows, int max_cols, short2* xy,
-                      uint16_t* fr, size_t stride, int pitch, cudaStream_t stream);
+// The parameter row of one map: the raw camera `raw` the coefficients d belong to, the camera `cam` of the undistorted image,
+// the coefficients and the frame size
+#define VO_LENS_PAR 18
+void vo_lens_row(double row[VO_LENS_PAR], const VoIntrinsics& raw, const VoIntrinsics& cam, const double d[8], int cols, int rows);
+// map of image im = 0 .. n-1, all of lens model `model` (B200VO_LENS_*): cv2.initUndistortRectifyMap(K, d, None, Knew,
+// (cols, rows), CV_16SC2) or cv2.fisheye.initUndistortRectifyMap(K, d, I, Knew, ...), into xy / fr + im_of[im] * stride,
+// rows `pitch` entries apart.  par: [n] vo_lens_row rows.
+int vo_undistort_maps(b200vo_ctx* ctx, int model, const double* d_par, const int* d_im_of, int n, int max_rows, int max_cols,
+                      short2* xy, uint16_t* fr, size_t stride, int pitch, cudaStream_t stream);
 // raw frames z = 0 .. n-1 (rows of `row` bytes, `stride` apart) -> undistorted frames at dst (same layout).  Frame z is
 // image seq_of[z >> seq_shift] of ud (seq_of == nullptr: image z) at that image's size: ext[image] (nullptr: rows x cols).
 // An image without distortion is copied.

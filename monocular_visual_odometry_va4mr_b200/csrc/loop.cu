@@ -558,7 +558,15 @@ extern "C" int b200vo_loop_set_frame_size(b200vo_loop* lp, int n_seq, const int3
 extern "C" int b200vo_loop_set_distortion(b200vo_loop* lp, int n_seq, const int32_t* seqs, const double* dist)
 {
     bool stale = false;
-    const int rc = lp ? batch_set_distortion(lp->B, n_seq, seqs, dist, &stale) : B200VO_E_BADARG;
+    const int rc = lp ? batch_set_lens(lp->B, n_seq, seqs, nullptr, dist, nullptr, &stale) : B200VO_E_BADARG;
+    return stale ? loop_idle(lp, n_seq, seqs) : rc;
+}
+
+extern "C" int b200vo_loop_set_lens(b200vo_loop* lp, int n_seq, const int32_t* seqs, const int32_t* model, const double* coeffs,
+                                    const double* raw_K)
+{
+    bool stale = false;
+    const int rc = lp ? batch_set_lens(lp->B, n_seq, seqs, model, coeffs, raw_K, &stale) : B200VO_E_BADARG;
     return stale ? loop_idle(lp, n_seq, seqs) : rc;
 }
 

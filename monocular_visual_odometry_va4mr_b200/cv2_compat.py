@@ -406,24 +406,30 @@ def recoverPose(E, points1, points2, cameraMatrix=None, R=None, t=None, mask=Non
 
 
 # --------------------------------------------------------------------------------------
-# cv2.undistort  (raw frames of cameras with lens distortion)
+# cv2.undistort and cv2.fisheye.undistortImage  (raw frames of cameras with lens distortion)
 # --------------------------------------------------------------------------------------
+def _pinhole_arg(M, name, what):
+    """a 3 x 3 camera matrix argument: ``error`` unless 3 x 3, ``NotImplementedError`` unless a pinhole (no skew, last row
+    0 0 1); its other checks (fx, fy > 0, finite) are the library's"""
+    M = np.asarray(M, np.float64)
+    if M.shape != (3, 3):
+        raise error(f"b200vo {what}: (-215:Assertion failed) {name} is 3x3")
+    if M[0, 1] != 0 or M[1, 0] != 0 or M[2, 0] != 0 or M[2, 1] != 0 or M[2, 2] != 1:
+        raise NotImplementedError(f"b200vo {what}: only pinhole camera matrices (no skew, last row 0 0 1)")
+    return np.ascontiguousarray(M)
+
+
 def undistort(src, cameraMatrix, distCoeffs, dst=None, newCameraMatrix=None):
-    """cv2.undistort(src, cameraMatrix, distCoeffs) -> uint8 image of src's shape, byte for byte what cv2 computes.  src: 2-D
-    uint8.  distCoeffs: 4, 5 or 8 coefficients (k1, k2, p1, p2[, k3[, k4, k5, k6]]) or None (a copy).  newCameraMatrix
-    other than None or cameraMatrix, multi-channel images, the 12- and 14-coefficient models and a cameraMatrix with skew
-    raise ``NotImplementedError``; a bad cameraMatrix or non-finite coefficients raise ``error``."""
+    """cv2.undistort(src, cameraMatrix, distCoeffs, newCameraMatrix=) -> uint8 image of src's shape, byte for byte what cv2
+    computes.  src: 2-D uint8.  distCoeffs: 4, 5 or 8 coefficients (k1, k2, p1, p2[, k3[, k4, k5, k6]]) or None (a copy).
+    newCameraMatrix: the pinhole camera of the undistorted image (e.g. from ``cv2.getOptimalNewCameraMatrix``), None:
+    cameraMatrix.  Multi-channel images, the 12- and 14-coefficient models and camera matrices with skew or another last
+    row raise ``NotImplementedError``; a bad camera matrix or non-finite coefficients raise ``error``."""
     if isinstance(src, np.ndarray) and src.ndim == 3:
         raise NotImplementedError("b200vo undistort: single-channel images only")
     src, step = _image_arg(src, "src")
-    K = np.asarray(cameraMatrix, np.float64)
-    if K.shape != (3, 3):
-        raise error("b200vo undistort: (-215:Assertion failed) cameraMatrix is 3x3")
-    K = np.ascontiguousarray(K)
-    if newCameraMatrix is not None and not np.array_equal(np.asarray(newCameraMatrix, np.float64), K):
-        raise NotImplementedError("b200vo undistort: newCameraMatrix must be None or cameraMatrix")
-    if K[0, 1] != 0 or K[1, 0] != 0 or K[2, 0] != 0 or K[2, 1] != 0 or K[2, 2] != 1:
-        raise NotImplementedError("b200vo undistort: only pinhole camera matrices (no skew, last row 0 0 1)")
+    K = _pinhole_arg(cameraMatrix, "cameraMatrix", "undistort")
+    Kn = K if newCameraMatrix is None else _pinhole_arg(newCameraMatrix, "newCameraMatrix", "undistort")
     d = np.zeros(4) if distCoeffs is None else np.asarray(distCoeffs, np.float64).reshape(-1)
     if d.size in (12, 14):
         raise NotImplementedError("b200vo undistort: the thin-prism (12) and tilted (14) models are not supported")
@@ -432,13 +438,41 @@ def undistort(src, cameraMatrix, distCoeffs, dst=None, newCameraMatrix=None):
     d = np.ascontiguousarray(d)
     out = np.empty(src.shape, np.uint8)
     ctx = _ctx()
-    rc = ctx.lib.b200vo_undistort(ctx.h, _p(src, c_u8p), src.shape[0], src.shape[1], step, _p(K, c_f64p), _p(d, c_f64p), d.size,
-                                  _p(out, c_u8p))
+    rc = ctx.lib.b200vo_undistort_new_camera(ctx.h, _p(src, c_u8p), src.shape[0], src.shape[1], step, _p(K, c_f64p), _p(d, c_f64p),
+                                             d.size, _p(Kn, c_f64p), _p(out, c_u8p))
     if rc != 0:
         _raise(ctx, rc, "undistort")
     if dst is not None:
         dst[...] = out
         return dst
+    return out
+
+
+def fisheye_undistort_image(distorted, K, D, undistorted=None, Knew=None, new_size=None):
+    """cv2.fisheye.undistortImage(distorted, K, D, Knew=, new_size=) -> uint8 image of distorted's shape, byte for byte what
+    cv2 computes.  distorted: 2-D uint8.  D: the 4 coefficients k1, k2, k3, k4.  Knew: the pinhole camera of the undistorted
+    image (usually K, or ``cv2.fisheye.estimateNewCameraMatrixForUndistortRectify``'s); None is the identity, as in cv2.
+    Multi-channel images, camera matrices with skew or another last row and a new_size other than the image's raise
+    ``NotImplementedError``; a bad camera matrix, a D without 4 elements or non-finite coefficients raise ``error``."""
+    if isinstance(distorted, np.ndarray) and distorted.ndim == 3:
+        raise NotImplementedError("b200vo fisheye.undistortImage: single-channel images only")
+    src, step = _image_arg(distorted, "distorted")
+    K = _pinhole_arg(K, "K", "fisheye.undistortImage")
+    Kn = None if Knew is None else _pinhole_arg(Knew, "Knew", "fisheye.undistortImage")
+    if new_size is not None and tuple(new_size) not in ((0, 0), (src.shape[1], src.shape[0])):
+        raise NotImplementedError("b200vo fisheye.undistortImage: new_size must be the image's (width, height)")
+    d = np.ascontiguousarray(np.asarray(D, np.float64).reshape(-1))
+    if d.size != 4:
+        raise error("b200vo fisheye.undistortImage: (-215:Assertion failed) D.total() == 4")
+    out = np.empty(src.shape, np.uint8)
+    ctx = _ctx()
+    rc = ctx.lib.b200vo_fisheye_undistort(ctx.h, _p(src, c_u8p), src.shape[0], src.shape[1], step, _p(K, c_f64p), _p(d, c_f64p),
+                                          None if Kn is None else _p(Kn, c_f64p), _p(out, c_u8p))
+    if rc != 0:
+        _raise(ctx, rc, "fisheye.undistortImage")
+    if undistorted is not None:
+        undistorted[...] = out
+        return undistorted
     return out
 
 
